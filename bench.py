@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- bridge-bidding env-steps/sec (BASELINE.json metric) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sweep]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--sweep] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): random-legal-action env stepping, 8192 envs per
@@ -188,6 +188,22 @@ def _config(n_gpus):
             "l2": "trajectory written per step = 519 MB > 126 MB L2 (no flush needed)"}
 
 
+DUMP_ENVS = 512  # envs of the [32, 8192, ...] trajectory written by --dump-outputs: 34 MB in all
+
+
+def dump_outputs(out_dir, np, traj, actions, stats):
+    """What a caller of the timed path receives after its last step, as float32 / float64 .npy files, so that two builds
+    can be compared output for output.  The full observation trajectory is 503 MB, so every per-env array is cut to the
+    same fixed, seeded sample of DUMP_ENVS env columns (sorted); the statistics are the i64[4] sums over the timed steps."""
+    os.makedirs(out_dir, exist_ok=True)
+    cols = np.sort(np.random.default_rng(SEED).choice(traj.terminated.shape[1], DUMP_ENVS, replace=False))
+    arrays = {"observation": traj.observation, "legal_action_mask": traj.legal_action_mask, "rewards": traj.rewards,
+              "terminated": traj.terminated, "current_player": traj.current_player, "action": actions}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy()[:, cols].astype(np.float32))
+    np.save(os.path.join(out_dir, "episode_stats.npy"), stats.cpu().numpy().astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -200,6 +216,8 @@ def main():
     ap.add_argument("--no-update", action="store_true", help="skip the PPO-update leg (SURVEY 8f-1)")
     ap.add_argument("--no-matches", action="store_true", help="skip the configs[0] / [3] / [4] duplicate-match legs")
     ap.add_argument("--league", action="store_true", help="run the configs[4] 1M-env league leg below 8 GPUs too")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's trajectory, sampled; the statistics) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -287,6 +305,8 @@ def main():
     env_steps = n * k * args.steps * world
     value = env_steps / (total_ms * 1e-3)
     avg_kernel_ms = sum(kernel_ms) / len(kernel_ms)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np, traj, actions, sums)
     peak, peak_src = _peaks()
     achieved = BYTES_PER_ENV_STEP * n * k / (avg_kernel_ms * 1e-3) / 1e9
     traffic, traffic_src = _traffic("bench_rollout")
@@ -511,7 +531,7 @@ def run_e2e(torch, np, _lib, table_np, n, offset, dev, world, dist, steps, warmu
 
 
 def _weights(name):
-    """bundled model pickle shipped as a data fixture (tests/golden/_weights, copied by __graft_entry__.build())"""
+    """bundled model pickle of the reference (15 MB each, not in the repository) if copied to tests/golden/_weights"""
     path = os.path.join(ROOT, "tests", "golden", "_weights", name)
     return path if os.path.exists(path) else None
 

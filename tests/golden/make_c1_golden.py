@@ -1,9 +1,10 @@
 """Golden vectors for BASELINE.json configs[0]: the `eval.py` duplicate match
 `model-pretrained-rl.pkl` vs `model-sl.pkl`, num_eval_envs=100 (eval.py:28,43-65; src/evaluation.py:69-204).
 
-Run HERE (the container where /root/reference is mounted), not on the GPU box:
+Run where the reference tree is available (its path is the first argument):
 
-    python tests/golden/make_c1_golden.py
+    python tests/golden/make_c1_golden.py /path/to/reference            # -> c1_eval_match.npz
+    python tests/golden/make_c1_golden.py /path/to/reference --seeded   # -> c1_seeded_match.npz
 
 What it does
   * loads the two BUNDLED pickles (bridge_models/, real trained weights) without jax;
@@ -15,8 +16,9 @@ What it does
     format into `JsonParser`, `calc_score` and `score_to_imp` (wb5/analyze_log.py:63-155);
   * freezes per-step actions, liveness, float64 top-2 logit gaps (how close each decision is to a tie), per-board IMPs,
     both tables' final contracts and mean / SE / win-rate into tests/golden/c1_eval_match.npz;
-  * copies the five bundled weight files to tests/golden/_weights/ (git-ignored, travels to the GPU box with the snapshot
-    like the built .so) -- __graft_entry__.build() does the same copy.
+  * copies the five bundled weight files to tests/golden/_weights/ (git-ignored: 15 MB each).
+With --seeded the same match is played by the two seeded nets of tests/helpers.seeded_params (SEEDED_WEIGHTS) instead of
+the bundled pickles, so that the repository alone can check a whole match against the reference's scorer.
 """
 import os
 import shutil
@@ -27,18 +29,17 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
-REF_ENV = os.path.join(REF, "submodule", "bridge_env")
 WEIGHTS = os.path.join(HERE, "_weights")
 MODELS = ("model-pretrained-rl.pkl", "model-sl.pkl", "model-from-scratch-rl.pkl", "model-pretrained-rl-with-fsp.pkl",
           "model-pretrained-rl-with-pfsp.pkl")
+SEEDED_WEIGHTS = (1, 2)
 
 
-def copy_weights():
+def copy_weights(ref):
     os.makedirs(WEIGHTS, exist_ok=True)
     for name in MODELS:
         dst = os.path.join(WEIGHTS, name)
-        src = os.path.join(REF, "bridge_models", name)
+        src = os.path.join(ref, "bridge_models", name)
         if not os.path.exists(dst) or os.path.getsize(dst) != os.path.getsize(src):
             shutil.copyfile(src, dst)
 
@@ -50,15 +51,18 @@ def mlp64(p, x):
     return h @ p["w4"].astype(np.float64) + p["b4"].astype(np.float64)
 
 
-def main():
+def main(ref, seeded):
     from brl_b200 import board_log
     from brl_b200 import random as brandom
     from brl_b200.models import load_params, params_to_numpy
     from oracle import oracle as orc
     from tests import helpers as H
-    copy_weights()
-    p1 = params_to_numpy(load_params(os.path.join(WEIGHTS, MODELS[0]), "cpu"))
-    p2 = params_to_numpy(load_params(os.path.join(WEIGHTS, MODELS[1]), "cpu"))
+    if seeded:
+        p1, p2 = (params_to_numpy(H.seeded_params(s, "cpu")) for s in SEEDED_WEIGHTS)
+    else:
+        copy_weights(ref)
+        p1 = params_to_numpy(load_params(os.path.join(WEIGHTS, MODELS[0]), "cpu"))
+        p2 = params_to_numpy(load_params(os.path.join(WEIGHTS, MODELS[1]), "cpu"))
     boards = H.load_boards()
     n = 100
     rng = brandom.PRNGKey(0)                      # eval.py:44
@@ -91,7 +95,7 @@ def main():
                                            priv0["shuffled_players"], record, team_names=("team1", "team2"),
                                            board_ids=[str(i) for i in range(n)])
     import tempfile
-    sys.path.insert(0, REF_ENV)
+    sys.path.insert(0, os.path.join(ref, "submodule", "bridge_env"))
     from bridge_env import Pair, Player
     from bridge_env.data_handler.json_handler.parser import JsonParser
     from bridge_env.score import calc_score, score_to_imp
@@ -120,13 +124,16 @@ def main():
         a_last_bid=env.info_a["last_bid"].astype(np.int32), a_last_bidder=env.info_a["last_bidder"].astype(np.int32),
         a_rewards=env.info_a["rewards"].astype(np.float32), b_last_bid=env.info_b["last_bid"].astype(np.int32),
         b_last_bidder=env.info_b["last_bidder"].astype(np.int32), b_rewards=env.info_b["rewards"].astype(np.float32),
-        deal=priv0["deal"].astype(np.int32), dealer=priv0["dealer"].astype(np.int32),
-        models=np.array(MODELS[:2]))
-    np.savez_compressed(os.path.join(HERE, "c1_eval_match.npz"), **out)
+        deal=priv0["deal"].astype(np.int32), dealer=priv0["dealer"].astype(np.int32))
+    if seeded:
+        out["weight_seeds"] = np.array(SEEDED_WEIGHTS, np.int64)
+    else:
+        out["models"] = np.array(MODELS[:2])
+    np.savez_compressed(os.path.join(HERE, "c1_seeded_match.npz" if seeded else "c1_eval_match.npz"), **out)
     fin = g[np.isfinite(g)]
     print(f"C1 golden: {len(actions)} steps, {int(np.stack(lives).sum())} live decisions, IMP {mean:.4f} +- {se:.4f}, "
           f"win rate {win:.3f}; smallest top-2 gap {fin.min():.3e}, decisions with gap <= 1e-4: {(fin <= 1e-4).sum()}")
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1], "--seeded" in sys.argv[2:])

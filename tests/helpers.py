@@ -23,14 +23,28 @@ def load_c1():
     return {k: z[k] for k in z.files}
 
 
+def load_c1_seeded():
+    """the configs[0] match played by two seeded nets (tests/golden/make_c1_golden.py --seeded)"""
+    z = np.load(os.path.join(GOLDEN, "c1_seeded_match.npz"))
+    return {k: z[k] for k in z.files}
+
+
+def seeded_params(seed, device):
+    """A net of the bundled models' architecture from a seed: haiku's initialisation (models.init_params) with the policy
+    head scaled by 128 (exact in fp32), so that its logits have a trained net's magnitude and the top-2 gaps of a match
+    stay far above the forward's rounding error."""
+    from brl_b200.models import LAYERS, init_params
+    p = init_params(seed, device)
+    p[LAYERS[4]]["w"] *= 128
+    return p
+
+
 def weight_path(name):
-    """bundled model pickle shipped as a fixture (git-ignored; __graft_entry__.build() copies it from the reference)"""
+    """bundled model pickle (bridge_models/ of the reference, 15 MB each): not in the repository; copy it to
+    tests/golden/_weights/ (git-ignored) to run the checks that use it"""
     path = os.path.join(GOLDEN, "_weights", name)
     if not os.path.exists(path):
-        ref = os.path.join("/root/reference/bridge_models", name)
-        if os.path.exists(ref):
-            return ref
-        raise FileNotFoundError(f"{path} is missing: run `python __graft_entry__.py` (build) where /root/reference is mounted")
+        raise FileNotFoundError(f"{path} is missing")
     return path
 
 

@@ -1,12 +1,11 @@
 """CPU: board logs of a duplicate match (brl_b200/board_log.py) in the reference's JSON format.
 A match is played on the oracle env with random-legal actions; the written files are then read
-back (a) structurally, against the golden score table, and (b) -- when the reference tree is
-mounted (this container, not the GPU box) -- by the reference's OWN `JsonParser`, `calc_score`
-and `score_to_imp` following wb5/analyze_log.py:63-155, whose IMPs must equal the env's."""
+back (a) structurally, against the golden score table, and (b) against what the reference's OWN
+`JsonParser`, `calc_score` and `score_to_imp` (wb5/analyze_log.py:63-155) read from the same
+logs, frozen in tests/golden/board_log_ref.npz, whose IMPs must equal the env's."""
 import io
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -15,8 +14,6 @@ from brl_b200 import board_log
 from brl_b200 import deals
 from oracle import oracle as orc
 from tests import helpers as H
-
-REF_ENV = "/root/reference/submodule/bridge_env"
 
 
 def _play_match(n=200, seed=5):
@@ -90,53 +87,38 @@ def test_match_logs_roundtrip_and_scores():
         assert orc.imp(s1 + s2) == int(cum[i])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ENV), reason="reference tree not mounted (GPU box)")
-def test_reference_parser_and_analysis_accept_the_logs(tmp_path):
+def test_reference_parser_and_analysis_accept_the_logs():
+    """The logs of this match, as the reference's `JsonParser`, `calc_score` and `score_to_imp` read them
+    (wb5/analyze_log.py:63-155, scores oriented to team "actor"), are frozen in tests/golden/board_log_ref.npz by
+    tests/golden/make_board_log_golden.py.  The logs written now must say the same and give the env's IMPs."""
     boards, env, priv0, record, cum = _play_match(n=120, seed=8)
-    t1, t2 = board_log.match_to_board_logs(boards["table"], priv0["deal"], priv0["dealer"], priv0["vul"],
-                                           priv0["shuffled_players"], record, team_names=("actor", "opp"),
-                                           board_ids=[str(i) for i in range(120)])
-    for name, entries in (("t1.json", t1), ("t2.json", t2)):
-        with open(tmp_path / name, "w") as fh:
-            board_log.write_logs(fh, entries)
-    sys.path.insert(0, REF_ENV)
-    try:
-        from bridge_env.data_handler.json_handler.parser import JsonParser
-        from bridge_env.score import calc_score, score_to_imp
-        from bridge_env import Pair
-    finally:
-        sys.path.remove(REF_ENV)
-    parser = JsonParser()
-    with open(tmp_path / "t1.json") as fh:
-        data1 = parser.parse_board_logs(fh)
-    with open(tmp_path / "t2.json") as fh:
-        data2 = parser.parse_board_logs(fh)
-
-    def dda_score(d):                                  # wb5/analyze_log.py:131-147
-        if d.contract.is_passed_out():
-            return 0
-        return calc_score(d.contract, d.dda[d.declarer][d.contract.trump])
-
-    for i, (d1, d2) in enumerate(zip(data1, data2)):
-        s1, s2 = dda_score(d1), dda_score(d2)
-        # wb5/analyze_log.py:86-95 orients both scores to table 1's N/S team; here to team "actor"
-        from bridge_env import Player
-        actor_pair_1 = Pair.NS if d1.players[Player.N] == "actor" else Pair.EW
-        actor_pair_2 = Pair.NS if d2.players[Player.N] == "actor" else Pair.EW
-        if d1.declarer is not None and d1.declarer.pair is not actor_pair_1:
-            s1 = -s1
-        if d2.declarer is not None and d2.declarer.pair is not actor_pair_2:
-            s2 = -s2
-        assert score_to_imp(s1, s2) == int(cum[i]), f"board {i}"
-        assert [str(b) for b in d1.bid_history] == t1[i]["bid_history"]
+    logs = board_log.match_to_board_logs(boards["table"], priv0["deal"], priv0["dealer"], priv0["vul"],
+                                         priv0["shuffled_players"], record, team_names=("actor", "opp"),
+                                         board_ids=[str(i) for i in range(120)])
+    ref = np.load(os.path.join(H.GOLDEN, "board_log_ref.npz"))
+    written = []
+    for entries in logs:
+        buf = io.StringIO()
+        board_log.write_logs(buf, entries)
+        written.append(json.loads(buf.getvalue())["logs"])
+    for i in range(120):
+        assert int(ref["imp"][i]) == int(cum[i]), f"board {i}"
+        for t in range(2):
+            e = written[t][i]
+            assert " ".join(e["bid_history"]) == ref["bid_history"][t, i], f"board {i} table {t + 1}"
+            assert (e["declarer"] or "") == ref["declarer"][t, i], f"board {i} table {t + 1}"
+            if e["declarer"] is not None:
+                assert e["contract"] == ref["contract"][t, i], f"board {i} table {t + 1}"
+            actor_side = "NS" if e["players"]["N"] == "actor" else "EW"
+            assert e["scores"][actor_side] == int(ref["score"][t, i]), f"board {i} table {t + 1}"
 
 
 @pytest.mark.gpu
-def test_gpu_match_record_to_board_logs_and_reference_parser(tmp_path):
+def test_gpu_match_record_to_board_logs_and_reference_parser():
     """SURVEY 8f-4 on the GPU path: a duplicate match played by the CUDA kernels (`record=` of
     make_simple_duplicate_evaluate: per step the action and both tables' terminated flags), written as the reference's
-    JSON board logs.  The logs' own scores must give the GPU match's IMPs board by board; where the reference tree is
-    mounted its `JsonParser` + `calc_score` + `score_to_imp` (wb5/analyze_log.py:63-155) must agree too."""
+    JSON board logs.  The logs' own scores must give the GPU match's IMPs board by board, and so must the reference's
+    `calc_score` + `score_to_imp` (wb5/analyze_log.py:131-147) applied to the written logs."""
     import torch
     from brl_b200 import BridgeBidding
     from brl_b200 import random as brandom
@@ -168,28 +150,27 @@ def test_gpu_match_record_to_board_logs_and_reference_parser(tmp_path):
             else:
                 assert e["contract"].rstrip("X") == board_log.ACTION_STR[info_bid + 3]
     assert abs(mean - float(cum.astype(np.float64).mean())) < 1e-9
-    if not os.path.isdir(REF_ENV):
-        return  # GPU box: the structural check above is all that can run
-    for name, entries in (("t1.json", t1), ("t2.json", t2)):
-        with open(tmp_path / name, "w") as fh:
-            board_log.write_logs(fh, entries)
-    sys.path.insert(0, REF_ENV)
-    try:
-        from bridge_env import Pair, Player
-        from bridge_env.data_handler.json_handler.parser import JsonParser
-        from bridge_env.score import calc_score, score_to_imp
-    finally:
-        sys.path.remove(REF_ENV)
-    parsed = []
-    for name in ("t1.json", "t2.json"):
-        with open(tmp_path / name) as fh:
-            parsed.append(JsonParser().parse_board_logs(fh))
+    # the reference's scorer as frozen in the golden tables (calc_bid_score -> score_table.npy, score_to_imp(d, 0) ->
+    # imp_table.npy, tests/golden/make_golden.py): each written log's contract, vulnerability and double-dummy tricks
+    # scored as wb5/analyze_log.py:131-147 does, oriented to team "actor", must give the GPU match's IMPs board by board
+    score_tab, imp_tab = np.load(H.GOLDEN + "/score_table.npy"), np.load(H.GOLDEN + "/imp_table.npy")
 
-    def actor_score(d):
-        if d.contract.is_passed_out():
+    def actor_score(e):
+        if e["contract"] == "Passed_out":
             return 0
-        s = calc_score(d.contract, d.dda[d.declarer][d.contract.trump])
-        return s if d.declarer.pair is (Pair.NS if d.players[Player.N] == "actor" else Pair.EW) else -s
+        bid = board_log.ACTION_STR.index(e["contract"].rstrip("X")) - 3
+        doubled = len(e["contract"]) - len(e["contract"].rstrip("X"))
+        pair = "NS" if e["declarer"] in "NS" else "EW"
+        tricks = e["dda"][e["declarer"]][board_log.STRAINS[bid % 5]]
+        s = int(score_tab[bid, doubled, int(e["vulnerability"] in (pair, "Both")), tricks])
+        return s if e["players"][pair[0]] == "actor" else -s
 
-    for i, (d1, d2) in enumerate(zip(*parsed)):
-        assert score_to_imp(actor_score(d1), actor_score(d2)) == int(cum[i]), f"board {i}"
+    written = []
+    for entries in (t1, t2):
+        buf = io.StringIO()
+        board_log.write_logs(buf, entries)
+        written.append(json.loads(buf.getvalue())["logs"])
+    assert (imp_tab[:401] == -24).all() and (imp_tab[1200:] == 24).all()    # 24 IMPs from 4000 points on
+    for i, (e1, e2) in enumerate(zip(*written)):
+        d = min(max(actor_score(e1) + actor_score(e2), -8000), 8000)
+        assert int(imp_tab[(d + 8000) // 10]) == int(cum[i]), f"board {i}"

@@ -344,24 +344,20 @@ def test_league_evaluate_equals_separate_matches():
     assert len({round(r[0], 6) for r in res}) == n_models  # three different opponents, three different results
 
 
-def test_c1_eval_match_with_bundled_weights_reproduces_golden():
-    """BASELINE configs[0] / eval.py:43-65: model-pretrained-rl.pkl vs model-sl.pkl, num_eval_envs=100, on the GPU path
-    (tensor-core forward, duplicate_step kernel).  Every live decision must equal the frozen float64 decision (the
-    smallest top-2 gap of the match is 1.4e-3, far above the forward's 1e-5 error), and IMP mean +- SE, the per-board
-    IMPs and both tables' contracts must equal the golden values, which the reference's own scorer reproduced."""
+def test_c1_eval_match_with_seeded_weights_reproduces_golden():
+    """BASELINE configs[0] / eval.py:43-65 (num_eval_envs=100, the 1000 real boards) played by two seeded nets of the
+    bundled models' architecture (tests/helpers.seeded_params) on the GPU path (tensor-core forward, duplicate_step
+    kernel).  Every live decision must equal the frozen float64 decision (the smallest top-2 gap of the match is 3.7e-3,
+    far above the forward's 1e-5 error), and IMP mean +- SE, the per-board IMPs and both tables' contracts must equal
+    the golden values, which the reference's own scorer reproduced (tests/golden/make_c1_golden.py --seeded)."""
     from brl_b200 import BridgeBidding
     from brl_b200.evaluation import make_simple_duplicate_evaluate
-    from brl_b200.models import load_params
     from brl_b200 import random as brandom
-    g = H.load_c1()
+    g = H.load_c1_seeded()
     boards = H.load_boards()
     env = BridgeBidding(table=boards["table"], device=DEV)
     n = int(g["n"])
-    try:
-        paths = [H.weight_path(str(m)) for m in g["models"]]
-    except FileNotFoundError as exc:   # the weight fixtures travel with the snapshot like the built .so; a bare clone lacks them
-        pytest.skip(str(exc))
-    p1, p2 = (load_params(p, DEV) for p in paths)
+    p1, p2 = (H.seeded_params(int(s), DEV) for s in g["weight_seeds"])
     evaluate = make_simple_duplicate_evaluate(env, "relu", "DeepMind", "relu", "DeepMind", n)
     trace = []
     (mean, se, win), info_a, info_b, cum = evaluate(p1, p2, brandom.PRNGKey(int(g["seed"])), trace=trace)

@@ -151,11 +151,29 @@ def test_illegal_action_terminates_with_penalty():
 def test_c1_golden_match_replays_on_the_oracle():
     """configs[0] (eval.py: model-pretrained-rl vs model-sl, 100 envs): the frozen action sequence (made with a float64
     MLP and checked board by board against the reference's own JsonParser / calc_score / score_to_imp by
-    tests/golden/make_c1_golden.py) replayed through the C oracle gives the frozen IMPs, contracts and statistics; and
-    the oracle's fp32 NumPy MLP on the bundled weights takes the same decisions."""
+    tests/golden/make_c1_golden.py) replayed through the C oracle gives the frozen IMPs, contracts and statistics; and,
+    where the bundled weights have been copied in, the oracle's fp32 NumPy MLP on them takes the same decisions."""
+    from brl_b200.models import load_params, params_to_numpy
+    g = H.load_c1()
+    try:
+        nets = [params_to_numpy(load_params(H.weight_path(str(m)), "cpu")) for m in g["models"]]
+    except FileNotFoundError:
+        nets = None  # the bundled weights are not in the repository: the env-side replay below still runs
+    _replay_c1_on_the_oracle(g, nets)
+
+
+def test_c1_seeded_match_replays_on_the_oracle():
+    """The same match played by the two seeded nets of tests/helpers.seeded_params (tests/golden/make_c1_golden.py
+    --seeded, checked against the reference's own scorer): replayed through the C oracle it gives the frozen IMPs,
+    contracts and statistics, and the oracle's fp32 NumPy MLP on the seeded nets takes the same decisions."""
+    from brl_b200.models import params_to_numpy
+    g = H.load_c1_seeded()
+    _replay_c1_on_the_oracle(g, [params_to_numpy(H.seeded_params(int(s), "cpu")) for s in g["weight_seeds"]])
+
+
+def _replay_c1_on_the_oracle(g, nets):
     from brl_b200 import random as brandom
     from oracle import oracle as orc
-    g = H.load_c1()
     boards = H.load_boards()
     n = int(g["n"])
     _, sub = brandom.split(brandom.PRNGKey(int(g["seed"])))
@@ -164,11 +182,6 @@ def test_c1_golden_match_replays_on_the_oracle():
     priv = env.export_private()
     assert (priv["deal"] == g["deal"]).all() and (priv["dealer"] == g["dealer"]).all()
     env.duplicate_tables_from_state()
-    try:
-        from brl_b200.models import load_params, params_to_numpy
-        nets = [params_to_numpy(load_params(H.weight_path(str(m)), "cpu")) for m in g["models"]]
-    except FileNotFoundError:
-        nets = None  # fresh clone without the weight fixtures: the env-side replay below still runs
     cum = np.zeros(n)
     for t in range(g["actions"].shape[0]):
         e = env.export()
@@ -178,7 +191,7 @@ def test_c1_golden_match_replays_on_the_oracle():
             lg = np.where((e["current_player"] < 2)[:, None], orc.mlp_forward(nets[0], e["observation"])[0],
                           orc.mlp_forward(nets[1], e["observation"])[0])
             act, _ = orc.categorical(lg, e["legal_action_mask"], sample=False)
-            assert (act[live] == g["actions"][t][live]).all()      # smallest float64 top-2 gap of the match is 1.4e-3
+            assert (act[live] == g["actions"][t][live]).all()      # smallest float64 top-2 gap: 1.4e-3 (bundled), 3.7e-3 (seeded)
         env.duplicate_step(g["actions"][t].astype(np.int32))
         cum += env.export()["rewards"][:, 0]
     assert env.export()["terminated"].all()
