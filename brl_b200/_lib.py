@@ -10,13 +10,18 @@ import os
 
 from . import build as _build
 
+# Supervised-learning ops, bound on their first call() instead of in load(): a process that never trains with them (the
+# rollout and PPO loops, bench.py) then creates exactly the Python objects it created before they existed.  Binding them
+# eagerly moved the interpreter's garbage-collection schedule in bench.py so that its rollout leg measured 8 % slower on a
+# B200 (1000 W), with identical device code and identical timings under gc.disable().
+LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
     "brl_match_stats", "brl_state_fields", "brl_gather_reward", "brl_team_rows", "brl_mlp_pack", "brl_obs_to_bf16", "brl_mlp_forward", "brl_policy_act",
     "brl_policy_act_rows",
     "brl_ppo_loss", "brl_adam_clip", "brl_adam_apply", "brl_gather_rows", "brl_eval_act_log", "brl_eval_summary", "brl_mlp_pack_train", "brl_mlp_adam_step", "brl_ppo_grad",
-)
+) + LAZY_OPS
 HOST_API = ("brl_env_create", "brl_env_destroy", "brl_env_init_host", "brl_env_step_host", "brl_env_rollout_host",
             "brl_env_rollout_host_async", "brl_env_wait", "brl_env_trajectory", "brl_env_rollout_host_compact_async",
             "brl_env_rollout_host_compact", "brl_result16_decode")
@@ -33,6 +38,7 @@ F_ACCUMULATE = 0x0004
 F_OBS_U8 = 0x0010
 F_OBS_BF16 = 0x0020
 F_SAMPLE = 0x0040
+F_SL_CHECK = 0x0080
 F_QUAD_LAST = 0x0100
 F_MLP_BF16 = 0x0200
 F_EVAL_INDICATOR_BIDS = 0x0400
@@ -71,6 +77,14 @@ class BrlPpoParams(C.Structure):
 class BrlAdamParams(C.Structure):
     _fields_ = [("n", C.c_int64), ("step", C.c_int32), ("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float),
                 ("eps", C.c_float), ("max_grad_norm", C.c_float)]
+
+
+class BrlSlParams(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("ent_coef", C.c_float), ("flags", C.c_int32)]
+
+
+SL_ACC_BYTES = 128  # include/brl_b200.h BRL_SL_ACC_BYTES
+SL_OK, SL_ILLEGAL, SL_EARLY_END, SL_NOT_ENDED = 0, 1, 2, 3  # brl_sl_examples check status (BRL_SL_*)
 
 
 PPO_VALUE_CLIPPING, PPO_REWARD_SCALING, PPO_UNMASKED_POLICY, PPO_ILLEGAL_STAT = 1, 2, 4, 8
@@ -113,6 +127,8 @@ def load():
     except OSError as exc:
         raise BrlError(f"cannot load {path}: {exc}; there is no CPU fallback") from exc
     for name in OPS:
+        if name in LAZY_OPS:
+            continue
         fn = getattr(L, name)
         fn.restype = C.c_int32
         fn.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t]
@@ -130,6 +146,8 @@ def load():
     L.brl_xla_layout.argtypes = [C.c_char_p]
     L.brl_xla_unreported_failures.restype = C.c_longlong
     for name in XLA_LEGACY:
+        if name[:-4] in LAZY_OPS:
+            continue
         fn = getattr(L, name)
         fn.restype = None
         fn.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_char_p, C.c_size_t, C.c_void_p]
@@ -168,7 +186,14 @@ def load():
 def call(name: str, stream: int, buffers, params) -> None:
     """Invoke one stream-first op: buffers = iterable of device addresses (int) or None."""
     L = load()
+    fn = getattr(L, name)
+    if fn.argtypes is None:  # one of LAZY_OPS, first call: bind it and its XLA symbol
+        fn.restype = C.c_int32
+        fn.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_void_p, C.c_size_t]
+        xla = getattr(L, name + "_xla")
+        xla.restype = None
+        xla.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.c_char_p, C.c_size_t, C.c_void_p]
     arr = (C.c_void_p * len(buffers))(*[C.c_void_p(b) if b else None for b in buffers])
-    rc = getattr(L, name)(C.c_void_p(stream), arr, C.byref(params), C.sizeof(params))
+    rc = fn(C.c_void_p(stream), arr, C.byref(params), C.sizeof(params))
     if rc != 0:
         raise BrlError(f"{name} failed ({rc}): {L.brl_last_error().decode()}")

@@ -1102,3 +1102,151 @@ int32_t brl_debug_role_cycles(unsigned long long* out8, int reset) {
 #endif
 
 }  // extern "C"
+
+// ---- brl_sl_examples: supervised-learning examples (make_dataset, sl.py:100-117) ---------------------------------------
+// A tile kernel like k_produce: phase 1 replays one stored auction prefix per lane with env_reset / env_step, phase 2 is
+// the block's emit_block.  BRL_F_SL_CHECK replays every whole auction once and writes a status byte per trajectory.
+namespace brl {
+
+// The dataset's deals: OpenSpiel's bridge(use_double_dummy_result=false) (sl.py:44) has dealer North, nobody vulnerable,
+// and players identical to seats.
+constexpr uint32_t kSlSeating = 0u | (1u << 2) | (2u << 4) | (3u << 6);
+constexpr uint32_t kTagSl = 0x534C3030u;  // "SL00": Philox stream of the call positions
+
+struct SlArgs {
+    const uint8_t* table;      // one 48-byte deal row per trajectory
+    const uint8_t* calls;      // call actions 0..37, trajectory t at [offsets[t], offsets[t + 1])
+    const int64_t* offsets;    // [n_traj + 1]
+    const int32_t* traj;       // [B]
+    const int32_t* position;   // [B] or NULL: uniform in [0, n_calls) from Philox(seed; example, step)
+    void* obs;
+    uint8_t* mask;
+    int32_t* label;
+    int32_t* position_out;     // optional
+    uint8_t* status;           // check mode: [n_traj]
+    int64_t n, env_offset, n_traj;
+    uint64_t seed;
+    uint32_t step;
+    int mask_vec;
+};
+
+__device__ __forceinline__ void sl_reset(Env& e, uint32_t t) { env_reset(e, t, 0u, 0u, 0u, kSlSeating, 0ull); }
+
+// sl.py:106: np.random.randint(52, len(trajectory)) -- a call position uniform in [0, n_calls)
+__device__ __forceinline__ int32_t sl_position(uint64_t seed, uint64_t example, uint32_t step, int64_t n_calls) {
+    const uint32_t r = philox4x32(make_uint4((uint32_t)example, (uint32_t)(example >> 32), kTagSl, step),
+                                  make_uint2((uint32_t)seed, (uint32_t)(seed >> 32))).x;
+    return (int32_t)__umulhi(r, (uint32_t)n_calls);
+}
+
+template <int EPW, int OBS>
+__global__ void __launch_bounds__(256) k_sl_examples(const SlArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    WarpTile<EPW>& t = *reinterpret_cast<WarpTile<EPW>*>(smem_raw);
+    const int lane = (int)threadIdx.x;
+    const int64_t env_base = (int64_t)blockIdx.x * EPW;
+    const int n_valid = (int)((a.n - env_base) < (int64_t)EPW ? (a.n - env_base) : (int64_t)EPW);
+    if (lane < 2) t.M[EPW + lane] = 0ull;
+    const int64_t i = env_base + lane;
+    // phase 1: one example per lane
+    if (lane < EPW) {
+        if (lane < n_valid) {
+            const uint32_t tr = (uint32_t)a.traj[i];
+            const int64_t off = a.offsets[tr], n_calls = a.offsets[tr + 1] - off;
+            int32_t pos = a.position ? a.position[i] : sl_position(a.seed, (uint64_t)(a.env_offset + i), a.step, n_calls);
+            const bool in_range = pos >= 0 && pos < n_calls;
+            if (!in_range) pos = pos < 0 ? 0 : (int32_t)n_calls;  // label -1 marks a position outside the auction
+            Env e;
+            sl_reset(e, tr);
+            for (int32_t k = 0; k < pos; ++k) env_step(e, (int32_t)a.calls[off + k], TableRows{a.table}, -1.0f, 1.0f);
+            a.label[i] = in_range ? (int32_t)a.calls[off + pos] : -1;
+            if (a.position_out) a.position_out[i] = in_range ? pos : -1;
+            stage_env<EPW>(t, lane, e, TableRows{a.table}, f_cur_seat(e), a.obs != nullptr);
+        } else {
+            t.M[lane] = 0ull;
+        }
+    }
+    __syncthreads();
+    // phase 2: the block's warps expand the rows
+    emit_block<EPW, OBS>(t, (int)threadIdx.x, (int)blockDim.x, env_base, n_valid, a.obs, a.mask, a.mask_vec);
+}
+
+// check mode: replay the whole auction of trajectory i (one thread each)
+__global__ void __launch_bounds__(256) k_sl_check(const SlArgs a) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    const int64_t off = a.offsets[i], n_calls = a.offsets[i + 1] - off;
+    Env e;
+    sl_reset(e, (uint32_t)i);
+    uint8_t st = BRL_SL_OK;
+    for (int64_t k = 0; k < n_calls && st == BRL_SL_OK; ++k) {
+        const int32_t c = (int32_t)a.calls[off + k];
+        if (f_terminated(e)) st = BRL_SL_EARLY_END;
+        else if (c >= kNumActions || !((env_legal_mask(e) >> c) & 1ull)) st = BRL_SL_ILLEGAL;
+        else env_step(e, c, TableRows{a.table}, -1.0f, 1.0f);
+    }
+    if (st == BRL_SL_OK && !f_terminated(e)) st = BRL_SL_NOT_ENDED;
+    a.status[i] = st;
+}
+
+template <int EPW, int OBS>
+static void launch_sl_examples_inst(const SlArgs& a, cudaStream_t s) {
+    const unsigned grid = (unsigned)((a.n + EPW - 1) / EPW);
+    k_sl_examples<EPW, OBS><<<grid, 128, sizeof(WarpTile<EPW>), s>>>(a);
+}
+template <int OBS>
+static void launch_sl_examples_obs(const SlArgs& a, cudaStream_t s) {
+    // 8 examples per block below 65,536 (enough blocks for every SM at B = 10,000), 16 above (not tuned)
+    if (a.n < 65536) launch_sl_examples_inst<8, OBS>(a, s);
+    else launch_sl_examples_inst<16, OBS>(a, s);
+}
+
+}  // namespace brl
+
+extern "C" {
+
+int32_t brl_sl_examples(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;
+    const bool check = (p->flags & BRL_F_SL_CHECK) != 0;
+    if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_sl_examples: n_deals must be the number of trajectories (> 0)");
+    static const char* names[] = {"deal_table", "calls", "offsets", "traj", "position", "obs", "mask", "label", "position_out", "status"};
+    for (int k : {0, 1, 2})
+        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_sl_examples: buffer '%s' is NULL", names[k]);
+    if (reinterpret_cast<uintptr_t>(b[0]) & 15u) return fail(BRL_E_BUFFER, "brl_sl_examples: buffer 'deal_table' is not 16-byte aligned");
+    SlArgs a{};
+    a.table = static_cast<const uint8_t*>(b[0]);
+    a.calls = static_cast<const uint8_t*>(b[1]);
+    a.offsets = static_cast<const int64_t*>(b[2]);
+    a.n = p->n_envs;
+    a.n_traj = p->n_deals;
+    a.env_offset = p->env_offset;
+    a.seed = p->seed;
+    a.step = p->step;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (check) {
+        if (b[9] == nullptr) return fail(BRL_E_BUFFER, "brl_sl_examples: buffer 'status' is NULL");
+        if (a.n > a.n_traj) return fail(BRL_E_OPAQUE, "brl_sl_examples: check mode covers n_envs <= n_deals trajectories");
+        a.status = static_cast<uint8_t*>(b[9]);
+        k_sl_check<<<(unsigned)((a.n + 255) / 256), 256, 0, s>>>(a);
+        return check_launch("brl_sl_examples (check)");
+    }
+    for (int k : {3, 5, 6, 7})
+        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_sl_examples: buffer '%s' is NULL", names[k]);
+    if (reinterpret_cast<uintptr_t>(b[5]) & 15u) return fail(BRL_E_BUFFER, "brl_sl_examples: buffer 'obs' is not 16-byte aligned");
+    a.traj = static_cast<const int32_t*>(b[3]);
+    a.position = static_cast<const int32_t*>(b[4]);
+    a.obs = b[5];
+    a.mask = static_cast<uint8_t*>(b[6]);
+    a.label = static_cast<int32_t*>(b[7]);
+    a.position_out = static_cast<int32_t*>(b[8]);
+    a.mask_vec = (reinterpret_cast<uintptr_t>(b[6]) & 15u) == 0;  // one row per example: the run of a tile starts at 16 B
+    if (p->flags & BRL_F_OBS_U8) launch_sl_examples_obs<kObsU8>(a, s);
+    else if (p->flags & BRL_F_OBS_BF16) launch_sl_examples_obs<kObsBF16>(a, s);
+    else launch_sl_examples_obs<kObsF32>(a, s);
+    return check_launch("brl_sl_examples");
+}
+
+}  // extern "C"

@@ -662,7 +662,8 @@ struct OpSpec {
 };
 
 template <int kFBN>
-static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, int nmb, uint32_t* ready, unsigned long long* trace) {
+static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, int nmb, uint32_t* ready, unsigned long long* trace,
+                                const char* what) {
     using Cfg = FusedTrainCfg<kFBN>;
     FusedTrainArgs fa{};
     int tiles = 0;
@@ -687,7 +688,7 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
         if (ok && o.a_lo) ok = pair_map(&f.a, o.a_hi, o.a_lo, o.a_mn != 0, o.m_rows, o.lda, kBM);
         else if (ok) ok = o.a_mn ? make_map(&f.a, o.a_hi, (uint64_t)o.k_cols, (uint64_t)o.m_rows, (uint64_t)o.lda, 64)
                                  : make_map(&f.a, o.a_hi, (uint64_t)o.m_rows, (uint64_t)o.k_cols, (uint64_t)o.lda, kBM);
-        if (!ok) return fail(BRL_E_LAUNCH, "brl_ppo_grad: cuTensorMapEncodeTiled failed");
+        if (!ok) return fail(BRL_E_LAUNCH, "%s: cuTensorMapEncodeTiled failed", what);
         f.g = o.g;
         f.g.M = o.m_rows;
         f.g.k_blocks = (o.k_cols + kBK - 1) / kBK;
@@ -712,7 +713,7 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
     int& n_sm = n_sm_dev[device_slot()];
     if (n_sm == 0) {
         if (cudaFuncSetAttribute(k_train_fused<kFBN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
-            return fail(BRL_E_LAUNCH, "brl_ppo_grad: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
+            return fail(BRL_E_LAUNCH, "%s: cannot reserve %u bytes of shared memory", what, Cfg::kSmemBytes);
         int dev = 0;
         cudaGetDevice(&dev);
         if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
@@ -727,7 +728,7 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
     at.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &at;
     cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, k_train_fused<kFBN>, fa) != cudaSuccess) return check_launch("brl_ppo_grad (fused launch)");
+    if (cudaLaunchKernelEx(&cfg, k_train_fused<kFBN>, fa) != cudaSuccess) return check_launch(what);
     return BRL_OK;
 }
 
@@ -806,34 +807,80 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
         if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_ppo_grad: buffer '%s' is not 16-byte aligned", names[k]);
     if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad: cuTensorMapEncodeTiled not available from the driver");
     cudaStream_t s = (cudaStream_t)stream;
-    const int B = (int)p->batch;
+    // 3. loss head + its backward (src/update.py:97-162)
+    struct PpoHead {
+        void** b;
+        BrlPpoParams params;
+        bool defer_illegal;
+    };
+    PpoHead head{b, *p, p->illegal_l2_coef == 0.0f};  // only the logged statistic needs the spectral norm: off the critical path
+    head.params.flags &= (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
+    head.params.reserved = 0;
+    const bool skip_illegal = head.defer_illegal && !(p->flags & BRL_PPO_ILLEGAL_STAT);  // statistic not asked for: stats[6] = NaN
+    auto ppo_head = [](cudaStream_t st, const TrainHeadIO& io, const void* ctx) -> int32_t {
+        const PpoHead& h = *static_cast<const PpoHead*>(ctx);
+        void* loss_buffers[13] = {const_cast<float*>(io.logits), const_cast<float*>(io.value), h.b[3], h.b[4], h.b[5], h.b[6], h.b[7],
+                                  h.b[8], h.b[9], io.dlogits, io.dvalue, h.b[11], h.b[12]};
+        return launch_ppo_loss(st, loss_buffers, &h.params, io.dz_hi, io.dz_lo, /*acc_zeroed=*/true, h.defer_illegal);
+    };
+    TrainMinibatch t{};
+    t.obs = b[0];
+    t.obs_flags = p->flags & (BRL_PPO_OBS_U8 | BRL_PPO_OBS_BF16);
+    t.index = static_cast<const int32_t*>(b[3]);
+    t.batch = p->batch;
+    t.blob = static_cast<const unsigned char*>(b[1]);
+    t.scratch = static_cast<unsigned char*>(b[2]);
+    t.grads = static_cast<float*>(b[10]);
+    t.grad_sumsq = static_cast<double*>(b[12]) + 14;  // |grads|^2 accumulates in acc[14] (input of brl_adam_apply)
+    t.zero = b[12];
+    t.zero_bytes = 16 * sizeof(double);
+    t.tune = p->reserved;
+    // deferred illegal-action statistic: its Gram tail runs in a spare block of the bias sums (gram_args reads only the
+    // logits / index / mask / scratch slots of the loss buffers)
+    GramArgs gram{};
+    if (head.defer_illegal && !skip_illegal) {
+        const TrainScratch S = train_scratch(p->batch);
+        void* loss_buffers[13] = {t.scratch + S.logits, nullptr, b[3], b[4], nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, b[11], b[12]};
+        gram = gram_args(loss_buffers, &head.params, static_cast<float*>(b[11]) + 6);
+        t.gram = &gram;
+        t.n_gram = gram_blocks(p->batch, 1024);
+    }
+    t.what = "brl_ppo_grad";
+    t.loss_head = ppo_head;
+    t.ctx = &head;
+    return launch_train_minibatch(s, t);
+}
+
+}  // extern "C"
+
+int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
+    const int B = (int)t.batch;
     const TrainBlob T = train_blob();
     const FlatLayout F = flat_layout();
     const TrainScratch S = train_scratch(B);
-    const unsigned char* blob = static_cast<const unsigned char*>(b[1]);
-    unsigned char* sc = static_cast<unsigned char*>(b[2]);
-    float* grads = static_cast<float*>(b[10]);
+    const unsigned char* blob = t.blob;
+    unsigned char* sc = t.scratch;
+    float* grads = t.grads;
     auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(sc + off); };
     int32_t rc = BRL_OK;
 
     // 0. counters and accumulators first, so that nothing but kernels (launched with programmatic dependent launch) follows
     if (cudaMemsetAsync(sc + S.ready, 0, ready_words(B) * sizeof(uint32_t), s) != cudaSuccess ||
-        cudaMemsetAsync(b[12], 0, 16 * sizeof(double), s) != cudaSuccess)
-        return check_launch("brl_ppo_grad (memset)");
+        (t.zero != nullptr && cudaMemsetAsync(t.zero, 0, t.zero_bytes, s) != cudaSuccess))
+        return check_launch(t.what);
     // 1. minibatch gather of the observation (src/update.py:194-199, cast of src/update.py:95)
     {
         const unsigned grid = (unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256);
-        const int32_t* index = static_cast<const int32_t*>(b[3]);
         uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
-        if (p->flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs<__nv_bfloat16>, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(b[0]), index, (int64_t)B, o);
-        else if (p->flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs<uint8_t>, dim3(grid), dim3(256), 0, s, static_cast<const uint8_t*>(b[0]), index, (int64_t)B, o);
-        else launch_pdl(k_gather_obs<float>, dim3(grid), dim3(256), 0, s, static_cast<const float*>(b[0]), index, (int64_t)B, o);
+        if (t.obs_flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs<__nv_bfloat16>, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(t.obs), t.index, (int64_t)B, o);
+        else if (t.obs_flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs<uint8_t>, dim3(grid), dim3(256), 0, s, static_cast<const uint8_t*>(t.obs), t.index, (int64_t)B, o);
+        else launch_pdl(k_gather_obs<float>, dim3(grid), dim3(256), 0, s, static_cast<const float*>(t.obs), t.index, (int64_t)B, o);
     }
     // 2. the GEMMs.  Forward: layers 1..4 (activations kept, row-major bf16 hi / lo: next layer's A, the ReLU mask, the
     //    wgrad's MN-major A) + the head.  Backward: dgrad into layer l's pre-activation, dz_l = (dz_{l+1} . W_{l+1}^T) * [h_l > 0]
     //    (S.dz_*[l-1], l = 1..4), and the wgrads dW_l = h_{l-1}^T . dz_l straight from the row-major h and dz.
-    // |grads|^2 accumulates in acc[14] (zeroed with the rest of acc by the loss head, which runs before every wgrad)
-    double* grad_sumsq = static_cast<double*>(b[12]) + 14;
+    // |grads|^2 accumulates in t.grad_sumsq (cleared by the caller before the loss head, which runs before every wgrad)
+    double* grad_sumsq = t.grad_sumsq;
     OpSpec fwd[5], bwd[kMaxOps];
     for (int l = 0; l < 5; ++l) {  // forward: A = previous activation (K-major), W = Wn[l] [in, out_pad] (MN-major)
         OpSpec& o = fwd[l];
@@ -909,39 +956,38 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
     }
     const int nmb = ready_blocks(B);
     uint32_t* ready = reinterpret_cast<uint32_t*>(sc + S.ready);
-    unsigned long long* trace = (p->reserved & 8) ? reinterpret_cast<unsigned long long*>(sc + S.trace) : nullptr;  // tune bit 3
+    unsigned long long* trace = (t.tune & 8) ? reinterpret_cast<unsigned long long*>(sc + S.trace) : nullptr;  // tune bit 3
     // Tile widths, measured on B200 at B = 1024 (scripts/exp_train_trace.py): the forward is a chain of layers with one tile
     // per SM per layer, where 128 x 64 tiles win; the backward has two independent GEMMs per layer (dgrad, wgrad) to fill the
     // SMs, where 128 x 128 tiles move a third fewer operand bytes.  Tune bit 2 / bit 4 flip them.
-    const bool wide_fwd = (p->reserved & 4) != 0, wide_bwd = (p->reserved & 16) == 0;
-    rc = wide_fwd ? launch_fused_ops<128>(s, fwd, 5, nmb, ready, trace) : launch_fused_ops<64>(s, fwd, 5, nmb, ready, trace);
+    const bool wide_fwd = (t.tune & 4) != 0, wide_bwd = (t.tune & 16) == 0;
+    rc = wide_fwd ? launch_fused_ops<128>(s, fwd, 5, nmb, ready, trace, t.what) : launch_fused_ops<64>(s, fwd, 5, nmb, ready, trace, t.what);
     if (rc != BRL_OK) return rc;
-    if ((rc = check_launch("brl_ppo_grad (forward)")) != BRL_OK) return rc;
-    // 3. loss head + its backward (src/update.py:97-162)
-    void* loss_buffers[13] = {sc + S.logits, sc + S.value, b[3], b[4], b[5], b[6], b[7], b[8], b[9], sc + S.dlogits, sc + S.dvalue, b[11], b[12]};
-    BrlPpoParams loss_params = *p;
-    loss_params.flags &= (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
-    loss_params.reserved = 0;
-    const bool defer_illegal = p->illegal_l2_coef == 0.0f;  // only the logged statistic needs the spectral norm: off the critical path
-    const bool skip_illegal = defer_illegal && !(p->flags & BRL_PPO_ILLEGAL_STAT);  // statistic not asked for: stats[6] = NaN
-    if ((rc = launch_ppo_loss(s, loss_buffers, &loss_params, sc + S.dz5_hi, sc + S.dz5_lo, /*acc_zeroed=*/true, defer_illegal)) != BRL_OK)
-        return rc;
+    if ((rc = check_launch(t.what)) != BRL_OK) return rc;
+    // 3. the caller's loss head (and its backward into d loss / d (logits, value))
+    TrainHeadIO io{};
+    io.logits = reinterpret_cast<const float*>(sc + S.logits);
+    io.value = reinterpret_cast<const float*>(sc + S.value);
+    io.dlogits = reinterpret_cast<float*>(sc + S.dlogits);
+    io.dvalue = reinterpret_cast<float*>(sc + S.dvalue);
+    io.dz_hi = sc + S.dz5_hi;
+    io.dz_lo = sc + S.dz5_lo;
+    if ((rc = t.loss_head(s, io, t.ctx)) != BRL_OK) return rc;
+    if (grads == nullptr) return BRL_OK;
     // 4. backward GEMMs
-    rc = wide_bwd ? launch_fused_ops<128>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr)
-                  : launch_fused_ops<64>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr);
+    rc = wide_bwd ? launch_fused_ops<128>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr, t.what)
+                  : launch_fused_ops<64>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr, t.what);
     if (rc != BRL_OK) return rc;
     // 5. bias gradients
     {
         BiasArgs a{};
         for (int l = 0; l < 4; ++l) { a.hi[l] = bf(S.dz_hi[l]); a.lo[l] = bf(S.dz_lo[l]); }
-        a.dlogits = reinterpret_cast<const float*>(sc + S.dlogits);
-        a.dvalue = reinterpret_cast<const float*>(sc + S.dvalue);
+        a.dlogits = io.dlogits;
+        a.dvalue = io.dvalue;
         a.grads = grads; a.sumsq = grad_sumsq; a.B = B; a.F = F;
-        a.n_gram = (defer_illegal && !skip_illegal) ? gram_blocks(B, 1024) : 0;
-        if (a.n_gram) a.gram = gram_args(loss_buffers, &loss_params, static_cast<float*>(b[11]) + 6);
+        a.n_gram = t.gram ? t.n_gram : 0;
+        if (a.n_gram) a.gram = *t.gram;
         launch_pdl(k_bias_grad, dim3(4 * (kHidden / 64) + 1 + (a.n_gram ? 1 : 0)), dim3(1024), 0, s, a);
     }
-    return check_launch("brl_ppo_grad");
+    return check_launch(t.what);
 }
-
-}  // extern "C"

@@ -63,6 +63,37 @@ struct GramArgs;
 GramArgs gram_args(void** loss_buffers, const BrlPpoParams* p, float* stat);
 int gram_blocks(int64_t batch, int threads);
 
+// One minibatch through the DeepMind MLP on tcgen05 (brl_mlp_train.cu), shared by brl_ppo_grad and brl_sl_grad /
+// brl_sl_eval: gather of the observation, fused forward with the activations kept, the caller's loss head, then (when
+// `grads` is set) the fused backward and the bias sums.  The ops differ only in the loss head.
+struct TrainHeadIO {  // what the forward leaves for the loss head, and where the backward reads d loss / d (logits, value)
+    const float* logits;  // f32 [B, 38]
+    const float* value;   // f32 [B]
+    float* dlogits;       // f32 [B, 38] (the head's bias sums read it)
+    float* dvalue;        // f32 [B]
+    void* dz_hi;          // bf16 hi / lo [B, 64]: 38 logits, value, zeros (the head's dgrad / wgrad operand)
+    void* dz_lo;
+};
+struct TrainMinibatch {
+    const void* obs;             // [total, 480] f32, or u8 / bf16 with obs_flags BRL_PPO_OBS_U8 / BRL_PPO_OBS_BF16
+    int32_t obs_flags;
+    const int32_t* index;        // [B] rows of obs, NULL = identity
+    int64_t batch;
+    const unsigned char* blob;   // brl_mlp_pack_train
+    unsigned char* scratch;      // brl_mlp_train_scratch_bytes(batch)
+    float* grads;                // flat fp32 gradient, NULL = forward and loss head only
+    double* grad_sumsq;          // += |grads|^2, or NULL
+    void* zero;                  // caller's accumulators, cleared together with the tile counters (NULL = none)
+    size_t zero_bytes;
+    int32_t tune;                // BrlPpoParams.reserved bits
+    const GramArgs* gram;        // deferred illegal-probability statistic, tail run in a spare block of the bias sums
+    int n_gram;                  // (0 = none)
+    const char* what;            // op name for error messages
+    int32_t (*loss_head)(cudaStream_t, const TrainHeadIO&, const void* ctx);
+    const void* ctx;
+};
+int32_t launch_train_minibatch(cudaStream_t stream, const TrainMinibatch& t);
+
 // Programmatic dependent launch for the short kernels of a dependent chain (the PPO optimizer step): the kernel may be
 // scheduled while its predecessor in the stream drains; it must execute pdl_wait() before touching global memory and
 // should call pdl_trigger() first so that ITS successor can be scheduled early too.

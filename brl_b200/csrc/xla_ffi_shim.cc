@@ -68,6 +68,9 @@
     X(brl_mlp_pack_train, "io") \
     X(brl_mlp_adam_step, "xixxix") \
     X(brl_ppo_grad, "iisiiiiiiioos") \
+    X(brl_sl_examples, "iiiiiooooo") \
+    X(brl_sl_grad, "iisiioos") \
+    X(brl_sl_eval, "iisiios") \
     /* end */
 
 namespace {

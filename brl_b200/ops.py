@@ -395,6 +395,59 @@ def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, a
                            _ptr(old_value), _ptr(adv), _ptr(targets), _ptr(grads), _ptr(stats), _ptr(acc)], p)
 
 
+def sl_examples(table, calls, offsets, traj, obs, mask, label, *, position=None, position_out=None, seed=0, step=0,
+                env_offset=0) -> None:
+    """make_dataset of sl.py:100-117 for a batch: example b replays trajectory traj[b] up to its call `position[b]` (drawn
+    uniformly in-kernel from Philox(seed; env_offset + b, step) when `position` is None) and gets the observation and
+    legal mask of the player to act, and that call as its label.  `obs` dtype: float32, uint8 / bool or bfloat16."""
+    if offsets.dtype != torch.int64 or calls.dtype != torch.uint8 or traj.dtype != torch.int32:
+        raise _lib.BrlError("sl_examples: calls must be uint8, offsets int64, traj int32")
+    n_traj = int(offsets.shape[0]) - 1
+    flags = obs_flag(obs.dtype)
+    _call("brl_sl_examples", [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(traj), _ptr(position), _ptr(obs), _ptr(mask),
+                              _ptr(label), _ptr(position_out), None],
+          _params(traj.shape[0], flags=flags, seed=seed, step=step, env_offset=env_offset, n_deals=n_traj))
+
+
+def sl_check(table, calls, offsets, status: torch.Tensor) -> None:
+    """Replay every whole auction once: status[t] = _lib.SL_OK / SL_ILLEGAL / SL_EARLY_END / SL_NOT_ENDED."""
+    n_traj = int(offsets.shape[0]) - 1
+    _call("brl_sl_examples", [_ptr(table), _ptr(calls), _ptr(offsets), None, None, None, None, None, None, _ptr(status)],
+          _params(n_traj, flags=_lib.F_SL_CHECK, n_deals=n_traj))
+
+
+def sl_acc(device) -> torch.Tensor:
+    """f64[16] accumulators of sl_grad / sl_eval (element 14 = sum of squares of the gradient after sl_grad)"""
+    return torch.zeros(_lib.SL_ACC_BYTES // 8, dtype=torch.float64, device=device)
+
+
+def _sl_params(name, obs, mask, label, scratch, blob, ent_coef):
+    L = _lib.load()
+    B = int(label.shape[0])
+    if obs.dtype == torch.bool:
+        obs = obs.view(torch.uint8)
+    if label.dtype != torch.int32 or mask.dtype != torch.uint8:
+        raise _lib.BrlError(f"{name}: label must be int32 and mask uint8")
+    if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
+        raise _lib.BrlError(f"{name}: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
+    return obs, _lib.BrlSlParams(B, float(ent_coef), obs_flag(obs.dtype))
+
+
+def sl_grad(obs, blob, scratch, mask, label, grads, stats, acc, *, ent_coef=0.0) -> None:
+    """One minibatch of value_and_grad(loss) of sl.py:169-184 through the MLP on tcgen05 -> flat fp32 gradients and
+    stats[:5] = {total_loss, target_loss, entropy, accuracy, illegal_actions_prob} of the parameters before the step."""
+    obs, p = _sl_params("sl_grad", obs, mask, label, scratch, blob, ent_coef)
+    if grads.dtype != torch.float32 or grads.numel() != _lib.load().brl_mlp_num_params():
+        raise _lib.BrlError("sl_grad: grads must be the flat fp32 gradient buffer")
+    _call("brl_sl_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+
+
+def sl_eval(obs, blob, scratch, mask, label, stats, acc, *, ent_coef=0.0) -> None:
+    """sl_grad's statistics without the backward (accuracy, sl.py:186-194; test metrics, sl.py:288-301)."""
+    obs, p = _sl_params("sl_eval", obs, mask, label, scratch, blob, ent_coef)
+    _call("brl_sl_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(stats), _ptr(acc)], p)
+
+
 def gather_rows(src: torch.Tensor, index: torch.Tensor, dst: torch.Tensor) -> None:
     """dst[b] = src[index[b]] over the leading axis (minibatch take, src/update.py:194-199)."""
     row_bytes = src[0].numel() * src.element_size()

@@ -56,6 +56,9 @@
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
+ *   brl_sl_examples       make_dataset: replay of a stored auction prefix -> (obs, legal mask, label)   sl.py:87-117
+ *   brl_sl_grad           jax.value_and_grad(loss)(params, inputs, targets, legal_actions)             sl.py:169-184,205-206
+ *   brl_sl_eval           loss + accuracy + illegal-action probability, no gradient                     sl.py:169-194,288-301
  */
 #ifndef BRL_B200_H
 #define BRL_B200_H
@@ -93,6 +96,7 @@ typedef struct CUstream_st *brl_stream_t; /* == cudaStream_t */
 #define BRL_F_UNIFORM_U16   0x2000 /* brl_rollout_random / brl_env_rollout_host_compact*: caller-supplied uniforms are u16[K,n] */
 #define BRL_F_SEED_SALT     0x4000 /* brl_policy_act: buffers[8] = device u64 XORed into `seed` (replayed CUDA graphs draw fresh noise) */
 #define BRL_F_COUNT_DONE    0x8000 /* brl_gather_reward: buffers[3] u8 done[n], [4] inout u64 count += sum(done) (src/roll_out.py:85) */
+#define BRL_F_SL_CHECK      0x0080 /* brl_sl_examples: replay every whole auction once and write a status byte per trajectory */
 #define BRL_F_HOST_STAGED   0x0800 /* brl_env_create: never write results straight into pinned host buffers (always stage + copy) */
 
 /* tuning (0 = automatic): bits 16-17 envs per block of the one-launch kernels (1->8, 2->16, 3->32), bits 18-19 warps
@@ -338,6 +342,46 @@ int32_t brl_mlp_adam_step(brl_stream_t, void **buffers, const void *opaque, size
  *               element 14 = sum of squares of grads (the input of brl_adam_apply) */
 int32_t brl_ppo_grad(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- supervised bidding pre-training (sl.py): examples from stored auctions, cross-entropy step ---------------------- */
+/* Examples of the OpenSpiel bidding data (sl.py:87-117): one deal row per trajectory (deals.py format, DD nibbles unused),
+ * dealer North, nobody vulnerable, players = seats (bridge(use_double_dummy_result=false), sl.py:44).  The calls of
+ * trajectory t are calls[offsets[t] .. offsets[t + 1]) as actions 0..37 (0 Pass, 1 X, 2 XX, 3.. = 1C..7NT).
+ * opaque = BrlParams: n_envs = examples B (check mode: trajectories to check), n_deals = trajectories in the table,
+ *          flags = BRL_F_OBS_U8 / BRL_F_OBS_BF16 (f32 default) | BRL_F_SL_CHECK, seed / step / env_offset key the positions.
+ * buffers: [0] in deal_table[n_deals, 48]  [1] in u8 calls[]  [2] in i64 offsets[n_deals + 1]  [3] in i32 traj[B]
+ *          [4] in i32 position[B] (call index in [0, n_calls); NULL -> uniform from Philox(seed; env_offset + b, step))
+ *          [5] out obs[B,480] of the player to act after calls [0, position)  [6] out u8 mask[B,38]
+ *          [7] out i32 label[B] = the call at `position` (-1: position outside the auction)  [8] out i32 position[B] (NULL ok)
+ *          [9] out u8 status[n_envs] -- written ONLY with BRL_F_SL_CHECK (then [3..8] are not read or written):
+ *              BRL_SL_* for trajectory i's whole auction */
+#define BRL_SL_OK        0 /* legal throughout, ends with its last call */
+#define BRL_SL_ILLEGAL   1 /* a call that is not legal where it is made */
+#define BRL_SL_EARLY_END 2 /* the auction is over before its last call */
+#define BRL_SL_NOT_ENDED 3 /* the auction is not over after its last call */
+int32_t brl_sl_examples(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
+typedef struct BrlSlParams {
+    int64_t batch;         /* examples in this minibatch; 0 = an empty batch (no-op)      */
+    float ent_coef;        /* SLConfig.entropy_coef                                      */
+    int32_t flags;         /* BRL_F_OBS_U8 / BRL_F_OBS_BF16: dtype of obs (f32 default)   */
+} BrlSlParams;
+#define BRL_SL_ACC_BYTES 128 /* f64[16] accumulators of brl_sl_grad / brl_sl_eval; element 14 = sum of squares of grads */
+
+/* One minibatch of `jax.value_and_grad(loss, has_aux=True)` (sl.py:169-184, 205-206) through the DeepMind MLP on tcgen05
+ * (the forward / backward of brl_ppo_grad with a cross-entropy head):
+ *   target_loss = -mean(one_hot(label, 38) * log_softmax(logits)) (mean over B * 38 entries, unmasked softmax),
+ *   entropy of the softmax over the legal calls, total = target_loss - ent_coef * entropy; the value head gets no gradient.
+ * Follow with brl_mlp_adam_step, eps = 1e-8, max_grad_norm = 0 (optax.adam(learning_rate), sl.py:166).  opaque = BrlSlParams.
+ * buffers: [0] in obs[B,480]  [1] in blob (brl_mlp_pack_train)  [2] scratch[brl_mlp_train_scratch_bytes(B)]
+ *          [3] in u8 mask[B,38]  [4] in i32 label[B]  [5] out f32 grads[brl_mlp_num_params()]
+ *          [6] out f32 stats[8] = {total_loss, target_loss, entropy, accuracy, illegal_actions_prob, 0, 0, 0}
+ *          [7] scratch f64[16] (BRL_SL_ACC_BYTES, 16-byte aligned) */
+int32_t brl_sl_grad(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_sl_grad's forward and statistics without the backward (the post-update train accuracy, sl.py:279, and the test
+ * metrics, sl.py:288-301): accuracy = mean(argmax softmax(logits) == label), illegal_actions_prob = mean(softmax . ~legal).
+ * buffers: [0] in obs  [1] in blob  [2] scratch  [3] in u8 mask[B,38]  [4] in i32 label[B]  [5] out f32 stats[8]  [6] scratch f64[16] */
+int32_t brl_sl_eval(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- full evaluation statistics (src/evaluation.py:207-1032) ---------------------------------- */
 #define BRL_F_EVAL_INDICATOR_BIDS 0x0400 /* non-duplicate `evaluate`: bid histogram is .set(1), not += 1 (src/evaluation.py:345-354) */
 #define BRL_EVAL_ACC_COLS 76    /* per-env log row: ill[2] steps[2] passes[2] actor_bid[35] opp_bid[35] (team 1 first) */
@@ -406,6 +450,9 @@ void brl_mlp_adam_step_xla(brl_stream_t, void **buffers, const char *opaque, siz
 void brl_ppo_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_act_log_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_summary_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_sl_examples_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_sl_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_sl_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------
  * Host-buffer convenience layer (the call a non-JAX host makes): the library
