@@ -10,11 +10,11 @@ import os
 
 from . import build as _build
 
-# Supervised-learning ops, bound on their first call() instead of in load(): a process that never trains with them (the
+# Supervised-learning and league ops, bound on their first call() instead of in load(): a process that never uses them (the
 # rollout and PPO loops, bench.py) then creates exactly the Python objects it created before they existed.  Binding them
 # eagerly moved the interpreter's garbage-collection schedule in bench.py so that its rollout leg measured 8 % slower on a
 # B200 (1000 W), with identical device code and identical timings under gc.disable().
-LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval")
+LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -27,7 +27,8 @@ HOST_API = ("brl_env_create", "brl_env_destroy", "brl_env_init_host", "brl_env_s
             "brl_env_rollout_host_compact", "brl_result16_decode")
 MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_scratch_bytes", "brl_mlp_rows_scratch_bytes",
         "brl_xla_layout", "brl_xla_unreported_failures", "brl_eval_num_sums",
-        "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset")
+        "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset",
+        "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 

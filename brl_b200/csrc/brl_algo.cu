@@ -153,6 +153,95 @@ __global__ void __launch_bounds__(1024) k_team_rows(const int8_t* __restrict__ p
     if (t2) rows2[base[1] + warp_cnt[1][warp] + __popc(b2 & below)] = (int32_t)i;
 }
 
+// ---- live-env grouping by acting net over a pool (workspace/eval_selfplay_league.py) ---------------------------
+// k_team_rows for many matches at once: env i is played by net env_models[i][0] for players 0/1 and env_models[i][1] for
+// players 2/3 (src/evaluation.py:124-151).  Count per net, lay the nets' groups out padded to kGroupRows rows, scatter.  The
+// envs of one match are contiguous, so a warp nearly always holds one or two nets: one atomic per net and warp.
+// A live env whose acting net id is outside [0, M) invalidates the grouping: offsets[M] (the count the host reads anyway to
+// size the forward) becomes -1, so the error surfaces before any forward runs, without an extra host read.
+constexpr int kNotListed = -1, kBadModel = -2;
+__device__ __forceinline__ int acting_model(const int8_t* player, const uint8_t* done, const int32_t* env_models, int64_t i,
+                                            int64_t n, int n_models) {
+    if (i >= n || (done != nullptr && done[i] != 0)) return kNotListed;
+    const int m = env_models[2 * i + (player[i] < 2 ? 0 : 1)];
+    return m >= 0 && m < n_models ? m : kBadModel;
+}
+
+__global__ void __launch_bounds__(256) k_model_count(const int8_t* __restrict__ player, const uint8_t* __restrict__ done,
+                                                     const int32_t* __restrict__ env_models, int32_t* __restrict__ counts,
+                                                     int32_t* __restrict__ offsets, int64_t n, int n_models) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int m = acting_model(player, done, env_models, i, n, n_models);
+    const unsigned peers = __match_any_sync(0xffffffffu, m);
+    if ((threadIdx.x & 31) != __ffs(peers) - 1) return;
+    if (m >= 0) atomicAdd(&counts[m], __popc(peers));
+    else if (m == kBadModel) offsets[n_models] = -1;  // zeroed before this launch; read by k_model_offsets
+}
+
+// one block: offsets[m] = sum of the padded sizes of nets < m, offsets[M] = padded total (or -1 when k_model_count met a bad
+// id); the block ids of each group, -1 in its padding rows; counts are reset to serve as the scatter's cursors (the scatter
+// brings them back to the counts)
+__global__ void __launch_bounds__(1024) k_model_offsets(int32_t* __restrict__ counts, int32_t* __restrict__ offsets,
+                                                        int32_t* __restrict__ block_model, int32_t* __restrict__ rows, int n_models) {
+    __shared__ int warp_sum[32];
+    __shared__ int carry, bad;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) {
+        carry = 0;
+        bad = offsets[n_models] < 0;
+    }
+    __syncthreads();
+    for (int c0 = 0; c0 < n_models; c0 += 1024) {
+        const int m = c0 + (int)threadIdx.x;
+        const int padded = m < n_models ? (counts[m] + kGroupRows - 1) / kGroupRows * kGroupRows : 0;
+        int incl = padded;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int v = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += v;
+        }
+        if (lane == 31) warp_sum[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            const int ws = warp_sum[lane];
+            int wi = ws;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, wi, o);
+                if (lane >= o) wi += v;
+            }
+            warp_sum[lane] = wi - ws;
+        }
+        __syncthreads();
+        const int off = carry + warp_sum[warp] + incl - padded;
+        if (m < n_models) {
+            offsets[m] = off;
+            const int cnt = counts[m];
+            for (int r = off + cnt; r < off + padded; ++r) rows[r] = -1;
+            for (int bl = off / kGroupRows; bl < (off + padded) / kGroupRows; ++bl) block_model[bl] = m;
+            counts[m] = 0;
+        }
+        __syncthreads();
+        if (threadIdx.x == 1023) carry = off + padded;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) offsets[n_models] = bad ? -1 : carry;
+}
+
+__global__ void __launch_bounds__(256) k_model_scatter(const int8_t* __restrict__ player, const uint8_t* __restrict__ done,
+                                                       const int32_t* __restrict__ env_models, const int32_t* __restrict__ offsets,
+                                                       int32_t* __restrict__ cursor, int32_t* __restrict__ rows, int64_t n, int n_models) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int m = acting_model(player, done, env_models, i, n, n_models);
+    const unsigned peers = __match_any_sync(0xffffffffu, m);
+    const int leader = __ffs(peers) - 1;
+    int base = 0;
+    if (m >= 0 && lane == leader) base = atomicAdd(&cursor[m], __popc(peers));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (m >= 0) rows[offsets[m] + base + __popc(peers & ((1u << lane) - 1u))] = (int32_t)i;
+}
+
 // ---- _imp_reward -- src/duplicate.py:15-70 ----------------------------------------------------
 __global__ void __launch_bounds__(256) k_imp_reward(const float4* __restrict__ a, const float4* __restrict__ b,
                                                     float4* __restrict__ out, int64_t n) {
@@ -189,6 +278,41 @@ __global__ void __launch_bounds__(256) k_match_stats(const float* __restrict__ x
         double t = 0.0;
         for (int k = 0; k < (int)(blockDim.x >> 5); ++k) t += sh[threadIdx.x][k];
         atomicAdd(&sums[threadIdx.x], t);
+    }
+}
+
+// the same sums over P contiguous env ranges [offsets[p], offsets[p + 1]) into sums[p][0..3] (the matches of a league
+// chunk); the grid's y dimension strides over the ranges, so P is not bounded by it.  The values are integer IMPs, so every
+// entry equals k_match_stats on that slice exactly.
+__global__ void __launch_bounds__(256) k_match_stats_ranges(const float* __restrict__ x, const int64_t* __restrict__ offsets,
+                                                            double* __restrict__ sums, int64_t n_ranges) {
+    __shared__ double sh[4][8];
+    for (int64_t p = blockIdx.y; p < n_ranges; p += gridDim.y) {
+        const int64_t lo = offsets[p], hi = offsets[p + 1];
+        double s1 = 0.0, s2 = 0.0, w = 0.0, c = 0.0;
+        for (int64_t i = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += (int64_t)gridDim.x * blockDim.x) {
+            double v = (double)x[i];
+            s1 += v;
+            s2 += v * v;
+            w += v > 0.0 ? 1.0 : 0.0;
+            c += 1.0;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+            s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+            w += __shfl_xor_sync(0xffffffffu, w, o);
+            c += __shfl_xor_sync(0xffffffffu, c, o);
+        }
+        int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+        if (lane == 0) { sh[0][warp] = c; sh[1][warp] = s1; sh[2][warp] = s2; sh[3][warp] = w; }
+        __syncthreads();
+        if (threadIdx.x < 4) {
+            double t = 0.0;
+            for (int k = 0; k < (int)(blockDim.x >> 5); ++k) t += sh[threadIdx.x][k];
+            if (t != 0.0) atomicAdd(&sums[8 * p + threadIdx.x], t);
+        }
+        __syncthreads();  // sh is reused by the next range
     }
 }
 
@@ -299,6 +423,55 @@ int32_t brl_match_stats(brl_stream_t stream, void** b, const void* opaque, size_
     k_match_stats<<<grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const float*>(b[0]), static_cast<double*>(b[1]),
                                                           p->n_envs);
     return check_launch("brl_match_stats");
+}
+
+int32_t brl_match_stats_ranges(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // no ranges: a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    BRL_REQUIRE(b[0], "x");
+    BRL_REQUIRE(b[1], "offsets");
+    BRL_REQUIRE(b[2], "sums");
+    const unsigned grid_y = (unsigned)(p->n_envs < 65535 ? p->n_envs : 65535);  // the kernel strides over the rest
+    k_match_stats_ranges<<<dim3(4u, grid_y), 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const float*>(b[0]), static_cast<const int64_t*>(b[1]), static_cast<double*>(b[2]), p->n_envs);
+    return check_launch("brl_match_stats_ranges");
+}
+
+int32_t brl_model_rows(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    const int64_t n_models = p->k_steps;
+    if (n_models <= 0) return fail(BRL_E_OPAQUE, "brl_model_rows: k_steps (the pool's model count) must be > 0");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (p->n_envs == 0) {  // an empty batch: every group is empty
+        if (b[4] != nullptr) cudaMemsetAsync(b[4], 0, n_models * sizeof(int32_t), s);
+        if (b[5] != nullptr) cudaMemsetAsync(b[5], 0, (n_models + 1) * sizeof(int32_t), s);
+        return check_launch("brl_model_rows");
+    }
+    BRL_REQUIRE(b[0], "current_player");
+    BRL_REQUIRE(b[2], "env_models");
+    BRL_REQUIRE(b[3], "rows");
+    BRL_REQUIRE(b[4], "counts");
+    BRL_REQUIRE(b[5], "offsets");
+    BRL_REQUIRE(b[6], "block_model");
+    if (p->n_envs > INT32_MAX / 2) return fail(BRL_E_OPAQUE, "brl_model_rows: n_envs too large");
+    int32_t* counts = static_cast<int32_t*>(b[4]);
+    if (cudaMemsetAsync(counts, 0, n_models * sizeof(int32_t), s) != cudaSuccess ||
+        cudaMemsetAsync(static_cast<int32_t*>(b[5]) + n_models, 0, sizeof(int32_t), s) != cudaSuccess)
+        return check_launch("brl_model_rows");
+    const unsigned grid = (unsigned)((p->n_envs + 255) / 256);
+    const int8_t* player = static_cast<const int8_t*>(b[0]);
+    const uint8_t* done = static_cast<const uint8_t*>(b[1]);
+    const int32_t* env_models = static_cast<const int32_t*>(b[2]);
+    k_model_count<<<grid, 256, 0, s>>>(player, done, env_models, counts, static_cast<int32_t*>(b[5]), p->n_envs, (int)n_models);
+    k_model_offsets<<<1, 1024, 0, s>>>(counts, static_cast<int32_t*>(b[5]), static_cast<int32_t*>(b[6]), static_cast<int32_t*>(b[3]),
+                                       (int)n_models);
+    k_model_scatter<<<grid, 256, 0, s>>>(player, done, env_models, static_cast<const int32_t*>(b[5]), counts,
+                                         static_cast<int32_t*>(b[3]), p->n_envs, (int)n_models);
+    return check_launch("brl_model_rows");
 }
 
 int32_t brl_gather_reward(brl_stream_t stream, void** b, const void* opaque, size_t len) {

@@ -22,6 +22,8 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
+#include <type_traits>
+
 #include "common.h"
 #include "env_device.cuh"
 #include "mlp_device.cuh"
@@ -252,6 +254,16 @@ struct LayerArgs {
     int M, n_total, k_blocks;
     int n_tiles_n, n_tiles;      // tiles along N, total tiles of this layer
 };
+// grouped forward (a pool of nets): rows [b * kGroupRows, (b + 1) * kGroupRows) use model block_model[b]; the pool's biases are
+// bias_stride floats apart; the grouped head runs the masked argmax of `act` in its epilogue.  A separate type, so that the
+// ungrouped kernels keep their parameter block (and their code) as it was.
+struct GroupedLayerArgs : LayerArgs {
+    const int32_t* block_model;
+    int64_t bias_stride;
+    ActArgs act;
+};
+template <bool GROUPED>
+using LayerArgsT = std::conditional_t<GROUPED, GroupedLayerArgs, LayerArgs>;
 
 template <int BN, bool SPLIT_A, bool SPLIT_W>
 struct LayerCfg {
@@ -261,10 +273,10 @@ struct LayerCfg {
     static constexpr uint32_t kSmemBytes = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD>
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
 __global__ void __launch_bounds__(kMlpThreads, 1)
 k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
-            const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, const LayerArgs a) {
+            const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, const LayerArgsT<GROUPED> a) {
     // PERSISTENT: one CTA per SM walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... (n-tile fastest, so the
     // CTAs running together share A row-blocks in L2).  The smem stage ring runs straight across tile
     // boundaries and the accumulator is double-buffered in TMEM, so the epilogue of tile j overlaps the
@@ -305,6 +317,8 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
             uint32_t it = 0;
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 const int m0 = (tile / n_tiles_n) * kBM, n0 = (tile % n_tiles_n) * BN;
+                int model = 0;
+                if constexpr (GROUPED) model = a.block_model[m0 / kGroupRows];
                 for (int kb = 0; kb < a.k_blocks; ++kb, ++it) {
                     const int s = (int)(it % S);
                     mbar_wait(empty_bar(s), ((it / S) & 1u) ^ 1u);
@@ -313,9 +327,14 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
                     tma_load_2d(dst, &tm_a_hi, full_bar(s), kb * kBK, m0);
                     dst += Cfg::kABytes;
                     if (SPLIT_A) { tma_load_2d(dst, &tm_a_lo, full_bar(s), kb * kBK, m0); dst += Cfg::kABytes; }
-                    tma_load_2d(dst, &tm_w_hi, full_bar(s), kb * kBK, n0);
-                    dst += Cfg::kWBytes;
-                    if (SPLIT_W) tma_load_2d(dst, &tm_w_lo, full_bar(s), kb * kBK, n0);
+                    if constexpr (GROUPED) {  // the pool's weights as {k, n, model}: this row block's net
+                        tma_load_3d(dst, &tm_w_hi, full_bar(s), kb * kBK, n0, model);
+                        if (SPLIT_W) tma_load_3d(dst + Cfg::kWBytes, &tm_w_lo, full_bar(s), kb * kBK, n0, model);
+                    } else {
+                        tma_load_2d(dst, &tm_w_hi, full_bar(s), kb * kBK, n0);
+                        dst += Cfg::kWBytes;
+                        if (SPLIT_W) tma_load_2d(dst, &tm_w_lo, full_bar(s), kb * kBK, n0);
+                    }
                 }
             }
         }
@@ -360,9 +379,12 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
             const int row = m0 + q * 32 + lane;
             const uint32_t t_row = tmem_acc + buf * BN + ((uint32_t)(q * 32) << 16);
             const float* bias = a.bias + n0;
-            if (!HEAD)
+            if constexpr (GROUPED) bias += (size_t)a.block_model[m0 / kGroupRows] * a.bias_stride;
+            if constexpr (!HEAD)
                 epilogue_hidden_row(t_row, BN, bias, row < a.M, a.out_hi + (size_t)row * a.n_total + n0,
                                     a.out_lo ? a.out_lo + (size_t)row * a.n_total + n0 : nullptr);
+            else if constexpr (GROUPED)  // padding rows of a group (row_index -1) are computed and dropped
+                epilogue_head_act_row(t_row, bias, row < a.M && a.act.row_index[row] >= 0, row, a.logits, nullptr, a.act);
             else
                 epilogue_head_row(t_row, bias, row < a.M, a.logits + (size_t)row * 38, a.value + row);
             // all of this warp's tcgen05.ld have completed (wait::ld): hand the accumulator back
@@ -400,6 +422,11 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap
     asm volatile(
         "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1, int c2) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+        ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
     asm volatile(
@@ -562,6 +589,12 @@ struct FusedArgs {
     int M, nmb, tiles_per_layer, n_tiles;
     ActArgs act;
 };
+struct GroupedFusedArgs : FusedArgs {  // grouped forward (see GroupedLayerArgs)
+    const int32_t* block_model;  // model of each kGroupRows-row block (= the CTA-pair tile height)
+    int64_t bias_stride;         // floats between two nets' biases in the pool
+};
+template <bool GROUPED>
+using FusedArgsT = std::conditional_t<GROUPED, GroupedFusedArgs, FusedArgs>;
 
 constexpr int kFusedBN = 256, kFusedTilesN = kHidden / kFusedBN;
 // Epilogue warps of the fused forward: TWO per TMEM lane quadrant, each draining half of the tile's 256 columns.  One
@@ -612,8 +645,16 @@ __device__ __forceinline__ unsigned long long mlp_now() {
 #define BRL_MLP_STAMP(tile, k)
 #endif
 
-template <bool SPLIT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_mlp_fused(const __grid_constant__ FusedArgs a) {
+// layer `layer`'s bias of row block `mb`'s net, and whether `row` is an env's row (padding rows of a group are dropped)
+__device__ __forceinline__ const float* fused_bias(const FusedArgs& a, int layer, int) { return a.bias[layer]; }
+__device__ __forceinline__ const float* fused_bias(const GroupedFusedArgs& a, int layer, int mb) {
+    return a.bias[layer] + (size_t)a.block_model[mb] * a.bias_stride;
+}
+__device__ __forceinline__ bool fused_row_ok(const FusedArgs& a, int row) { return row < a.M; }
+__device__ __forceinline__ bool fused_row_ok(const GroupedFusedArgs& a, int row) { return row < a.M && a.act.row_index[row] >= 0; }
+
+template <bool SPLIT, bool GROUPED = false>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_mlp_fused(const __grid_constant__ FusedArgsT<GROUPED> a) {
     using Cfg = FusedCfg<SPLIT>;
     constexpr int S = Cfg::kStages;
     constexpr uint32_t kTmemCols = 2 * kFusedBN;
@@ -677,6 +718,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
                     asm volatile("fence.proxy.async;" ::: "memory");  // generic-proxy writes -> async-proxy (TMA) reads
                 }
                 BRL_MLP_STAMP(tile, 1);
+                int model = 0;
+                if constexpr (GROUPED) model = a.block_model[f.mb];
                 for (int kb = 0; kb < k_blocks; ++kb, ++it) {
                     const int s = (int)(it % S);
                     mbar_wait(empty_bar(s), ((it / S) & 1u) ^ 1u);
@@ -686,8 +729,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
                     const uint32_t sw = sa + Cfg::kABytes * (SPLIT ? 2 : 1);
                     tma_load_2d_pair(sa, ma_hi, fb, kb * kBK, m0);
                     if (split_a) tma_load_2d_pair(sa + Cfg::kABytes, ma_lo, fb, kb * kBK, m0);
-                    tma_load_2d_pair(sw, mw_hi, fb, kb * kBK, n0);
-                    if (SPLIT) tma_load_2d_pair(sw + Cfg::kWBytes, mw_lo, fb, kb * kBK, n0);
+                    if constexpr (GROUPED) {  // the pool's weights as {k, n, model}: this row block's net
+                        tma_load_3d_pair(sw, mw_hi, fb, kb * kBK, n0, model);
+                        if (SPLIT) tma_load_3d_pair(sw + Cfg::kWBytes, mw_lo, fb, kb * kBK, n0, model);
+                    } else {
+                        tma_load_2d_pair(sw, mw_hi, fb, kb * kBK, n0);
+                        if (SPLIT) tma_load_2d_pair(sw + Cfg::kWBytes, mw_lo, fb, kb * kBK, n0);
+                    }
                 }
                 BRL_MLP_STAMP(tile, 2);
             }
@@ -744,16 +792,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
             if (f.layer < 4) {
                 const int n0 = f.nt * kFusedBN + half * kHalfCols;
                 if (SPLIT) {
-                    epilogue_hidden_tma(t_row + (uint32_t)(half * kHalfCols), kHalfCols, a.bias[f.layer] + n0, lane,
+                    epilogue_hidden_tma(t_row + (uint32_t)(half * kHalfCols), kHalfCols, fused_bias(a, f.layer, f.mb) + n0, lane,
                                         store_base + (uint32_t)(warp - 2) * 4096u, &a.st_hi[f.layer], &a.st_lo[f.layer], n0,
                                         m0 + q * 32);
                 } else {
                     __nv_bfloat16* oh = a.out_hi[f.layer];
-                    epilogue_hidden_row(t_row + (uint32_t)(half * kHalfCols), kHalfCols, a.bias[f.layer] + n0, row < a.M,
+                    epilogue_hidden_row(t_row + (uint32_t)(half * kHalfCols), kHalfCols, fused_bias(a, f.layer, f.mb) + n0, row < a.M,
                                         oh + (size_t)row * kHidden + n0, nullptr);
                 }
             } else if (half == 0) {  // the 64-column head tile: one warp per quadrant
-                epilogue_head_act_row(t_row, a.bias[4], row < a.M, row, a.logits, a.value, a.act);
+                epilogue_head_act_row(t_row, fused_bias(a, 4, f.mb), fused_row_ok(a, row), row, a.logits, a.value, a.act);
             }
             tc_fence_before();
             __syncwarp();  // orders the other lanes' activation stores before lane 0's fence (sync, one fence, one atomic)
@@ -779,19 +827,36 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
 }
 
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD>
+// a pool of nets (brl_policy_act_grouped): `n_models` packed blobs `stride` bytes apart, and the model of each kGroupRows-row block
+struct PoolArgs {
+    const int32_t* block_model;
+    int64_t stride;
+    int n_models;
+    ActArgs act;  // the per-layer head's masked argmax (the fused head takes launch_fused's `act`)
+};
+
+// weight operand of layer-tile loads: one net's [n_rows, k_in] bf16 matrix, or the pool's {k_in, n_rows, model} stack of them
+template <bool GROUPED>
+static bool make_w_map(CUtensorMap* m, const void* w, uint64_t n_rows, uint64_t k_in, uint32_t box_rows, const PoolArgs* pool) {
+    if constexpr (!GROUPED) return make_map(m, w, n_rows, k_in, k_in, box_rows);
+    const uint64_t dims[3] = {k_in, n_rows, (uint64_t)pool->n_models}, strides[2] = {k_in * 2, (uint64_t)pool->stride};
+    const uint32_t box[3] = {(uint32_t)kBK, box_rows, 1};
+    return make_map_nd(m, w, 3, dims, strides, box);
+}
+
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
 static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, int k_in, const void* w_hi, const void* w_lo,
-                            int n_valid_rows, const LayerArgs& args) {
+                            int n_valid_rows, const LayerArgs& args, const PoolArgs* pool = nullptr) {
     using Cfg = LayerCfg<BN, SPLIT_A, SPLIT_W>;
     CUtensorMap ta_hi, ta_lo, tw_hi, tw_lo;
     bool ok = make_map(&ta_hi, a_hi, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM) &&
-              make_map(&tw_hi, w_hi, (uint64_t)n_valid_rows, (uint64_t)k_in, (uint64_t)k_in, BN);
+              make_w_map<GROUPED>(&tw_hi, w_hi, (uint64_t)n_valid_rows, (uint64_t)k_in, BN, pool);
     ta_lo = ta_hi;
     tw_lo = tw_hi;
     if (ok && SPLIT_A) ok = make_map(&ta_lo, a_lo, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM);
-    if (ok && SPLIT_W) ok = make_map(&tw_lo, w_lo, (uint64_t)n_valid_rows, (uint64_t)k_in, (uint64_t)k_in, BN);
+    if (ok && SPLIT_W) ok = make_w_map<GROUPED>(&tw_lo, w_lo, (uint64_t)n_valid_rows, (uint64_t)k_in, BN, pool);
     if (!ok) return fail(BRL_E_LAUNCH, "brl_mlp_forward: cuTensorMapEncodeTiled failed");
-    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD>;
+    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED>;
     static bool attr_set_dev[kMaxDevices] = {};  // per device; idempotent, a race only repeats the call
     bool& attr_set = attr_set_dev[device_slot()];
     if (!attr_set) {
@@ -799,7 +864,13 @@ static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, 
             return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
         attr_set = true;
     }
-    LayerArgs la = args;
+    LayerArgsT<GROUPED> la{};
+    static_cast<LayerArgs&>(la) = args;
+    if constexpr (GROUPED) {
+        la.block_model = pool->block_model;
+        la.bias_stride = pool->stride / (int64_t)sizeof(float);
+        la.act = pool->act;
+    }
     la.n_tiles_n = (n_valid_rows + BN - 1) / BN;
     la.n_tiles = la.n_tiles_n * ((args.M + kBM - 1) / kBM);
     static int n_sm_dev[kMaxDevices] = {};
@@ -852,22 +923,23 @@ static int32_t launch_layer_pair(cudaStream_t s, const void* a_hi, const void* a
 // counters of the fused forward live behind the four activation buffers of the scratch
 static inline size_t fused_ready_bytes(int64_t n_envs) { return (size_t)(4 * 2 * ((n_envs + 2 * kBM - 1) / (2 * kBM))) * sizeof(uint32_t); }
 
-template <bool SPLIT>
+template <bool SPLIT, bool GROUPED = false>
 static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char* blob, const MlpLayout& L, __nv_bfloat16* const buf_hi[2],
-                            __nv_bfloat16* const buf_lo[2], uint32_t* ready, float* logits, float* value, int M, const ActArgs& act) {
+                            __nv_bfloat16* const buf_lo[2], uint32_t* ready, float* logits, float* value, int M, const ActArgs& act,
+                            const PoolArgs* pool = nullptr) {
     using Cfg = FusedCfg<SPLIT>;
-    FusedArgs fa{};
+    FusedArgsT<GROUPED> fa{};
     bool ok = true;
     for (int l = 0; l < 5 && ok; ++l) {
         const void* a_hi = l == 0 ? obs : (const void*)buf_hi[(l - 1) & 1];
         const void* a_lo = l == 0 ? obs : (const void*)buf_lo[(l - 1) & 1];
         const uint32_t w_box = l == 4 ? kHeadPad / 2 : kFusedBN / 2;
         ok = make_map(&fa.a_hi[l], a_hi, (uint64_t)M, (uint64_t)L.k_in[l], (uint64_t)L.k_in[l], kBM) &&
-             make_map(&fa.w_hi[l], blob + L.w_hi[l], (uint64_t)L.n_out[l], (uint64_t)L.k_in[l], (uint64_t)L.k_in[l], w_box);
+             make_w_map<GROUPED>(&fa.w_hi[l], blob + L.w_hi[l], (uint64_t)L.n_out[l], (uint64_t)L.k_in[l], w_box, pool);
         fa.a_lo[l] = fa.a_hi[l];
         fa.w_lo[l] = fa.w_hi[l];
         if (ok && SPLIT && l > 0) ok = make_map(&fa.a_lo[l], a_lo, (uint64_t)M, (uint64_t)L.k_in[l], (uint64_t)L.k_in[l], kBM);
-        if (ok && SPLIT) ok = make_map(&fa.w_lo[l], blob + L.w_lo[l], (uint64_t)L.n_out[l], (uint64_t)L.k_in[l], (uint64_t)L.k_in[l], w_box);
+        if (ok && SPLIT) ok = make_w_map<GROUPED>(&fa.w_lo[l], blob + L.w_lo[l], (uint64_t)L.n_out[l], (uint64_t)L.k_in[l], w_box, pool);
         fa.bias[l] = reinterpret_cast<const float*>(blob + L.bias[l]);
         if (l < 4) {
             fa.out_hi[l] = buf_hi[l & 1];
@@ -878,16 +950,20 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
         }
     }
     if (!ok) return fail(BRL_E_LAUNCH, "brl_mlp_forward: cuTensorMapEncodeTiled failed");
-    static_assert(sizeof(FusedArgs) <= 4096, "kernel parameters");
+    static_assert(sizeof(fa) <= 4096, "kernel parameters");
     fa.logits = logits;
     fa.value = value;
     fa.act = act;
     fa.ready = ready;
+    if constexpr (GROUPED) {
+        fa.block_model = pool->block_model;
+        fa.bias_stride = pool->stride / (int64_t)sizeof(float);
+    }
     fa.M = M;
     fa.nmb = (M + 2 * kBM - 1) / (2 * kBM);
     fa.tiles_per_layer = fa.nmb * kFusedTilesN;
     fa.n_tiles = 4 * fa.tiles_per_layer + fa.nmb;
-    auto kern = k_mlp_fused<SPLIT>;
+    auto kern = k_mlp_fused<SPLIT, GROUPED>;
     static int max_pairs_dev[kMaxDevices] = {};  // co-resident CTA pairs: the dependency waits need every launched pair to be running
     int& max_pairs = max_pairs_dev[device_slot()];
     if (max_pairs == 0) {
@@ -920,13 +996,20 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
     return BRL_OK;
 }
 
+// PADDED: index -1 marks a padding row of a grouped batch, gathered as zeros
+template <bool PADDED = false>
 __global__ void __launch_bounds__(256) k_gather_obs_rows(const uint4* __restrict__ src, const int32_t* __restrict__ index,
                                                          uint4* __restrict__ dst, int64_t n, int w) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n * w) return;
     const int64_t r = i / w;
     const int c = (int)(i - r * w);
-    dst[i] = src[(int64_t)index[r] * w + c];
+    if constexpr (PADDED) {
+        const int32_t e = index[r];
+        dst[i] = e >= 0 ? src[(int64_t)e * w + c] : make_uint4(0u, 0u, 0u, 0u);
+    } else {
+        dst[i] = src[(int64_t)index[r] * w + c];
+    }
 }
 
 }  // namespace brl
@@ -978,9 +1061,14 @@ int32_t brl_obs_to_bf16(brl_stream_t stream, void** b, const void* opaque, size_
     return check_launch("brl_obs_to_bf16");
 }
 
-// forward (+ optional fused categorical) shared by brl_mlp_forward and brl_policy_act
+}  // extern "C"
+
+// forward (+ optional fused categorical) shared by brl_mlp_forward and brl_policy_act.  GROUPED (brl_policy_act_grouped): `blob`
+// is a pool of nets, row block b of the batch runs net pool->block_model[b], and the head epilogue writes action / logits by env
+// (the per-layer head included: no categorical launch).  Its per-layer path has no CTA-pair variant (flags bit 28 is ignored).
+template <bool GROUPED = false>
 static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams* p, const void* obs, const unsigned char* blob,
-                                __nv_bfloat16* scratch, float* logits, float* value, const ActArgs& act) {
+                                __nv_bfloat16* scratch, float* logits, float* value, const ActArgs& act, const PoolArgs* pool = nullptr) {
     int32_t rc = BRL_OK;
     if (p->n_envs > (int64_t)1 << 30) return fail(BRL_E_OPAQUE, "%s: n_envs too large", who);
     if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "%s: cuTensorMapEncodeTiled not available from the driver", who);
@@ -995,8 +1083,8 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
     const bool fused = (p->flags & ((1 << 29) | (1 << 28))) ? false : ((p->flags & (1 << 30)) != 0 || M >= kPairMinM);
     if (fused) {
         uint32_t* ready = reinterpret_cast<uint32_t*>(scratch + 4 * act_elems);
-        rc = split ? launch_fused<true>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act)
-                   : launch_fused<false>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act);
+        rc = split ? launch_fused<true, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
+                   : launch_fused<false, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
         if (rc != BRL_OK) return rc;
         return check_launch(who);
     }
@@ -1020,37 +1108,39 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
             // these 1-CTA tiles): measured faster for the single-product mode and for large batches
             // (scripts/exp_mlp_ab.py); flags bit 26 / 27 force wide / narrow
             const bool wide = (p->flags & (1 << 27)) ? false : ((p->flags & (1 << 26)) != 0 || !split || M >= 32768);
-            const bool pair = (p->flags & (1 << 28)) != 0;
+            const bool pair = !GROUPED && (p->flags & (1 << 28)) != 0;
             if (pair) {
                 if (l == 0) rc = split ? launch_layer_pair<256, false, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
                                        : launch_layer_pair<256, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
                 else rc = split ? launch_layer_pair<256, true, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
                                 : launch_layer_pair<256, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
             } else if (wide) {
-                if (l == 0) rc = split ? launch_layer<256, false, true, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                                       : launch_layer<256, false, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
-                else rc = split ? launch_layer<256, true, true, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                                : launch_layer<256, false, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
-            } else if (l == 0) rc = split ? launch_layer<128, false, true, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                                   : launch_layer<128, false, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
-            else rc = split ? launch_layer<128, true, true, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                            : launch_layer<128, false, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
+                if (l == 0) rc = split ? launch_layer<256, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
+                                       : launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+                else rc = split ? launch_layer<256, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
+                                : launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            } else if (l == 0) rc = split ? launch_layer<128, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
+                                   : launch_layer<128, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else rc = split ? launch_layer<128, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
+                            : launch_layer<128, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
             in_hi = a.out_hi;
             in_lo = a.out_lo;
         } else {
-            a.logits = lg;
-            a.value = vl;
-            rc = split ? launch_layer<kHeadPad, true, true, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a)
-                       : launch_layer<kHeadPad, false, false, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a);
+            a.logits = GROUPED ? logits : lg;
+            a.value = GROUPED ? nullptr : vl;
+            rc = split ? launch_layer<kHeadPad, true, true, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool)
+                       : launch_layer<kHeadPad, false, false, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool);
         }
         if (rc != BRL_OK) return rc;
     }
     rc = check_launch(who);
-    if (rc != BRL_OK || act.action == nullptr) return rc;
+    if (GROUPED || rc != BRL_OK || act.action == nullptr) return rc;
     if (act.row_index && value != nullptr) return fail(BRL_E_OPAQUE, "%s: a row-indexed batch below the fused-launch size has no value output", who);
     return launch_categorical(s, lg, act.mask, act.action, act.log_prob, M, act.sample, act.seed, act.env_offset, act.step, act.row_index,
                               act.row_index ? logits : nullptr);
 }
+
+extern "C" {
 
 int32_t brl_mlp_forward(brl_stream_t stream, void** b, const void* opaque, size_t len) {
     int32_t rc;
@@ -1105,7 +1195,7 @@ int32_t brl_policy_act_rows(brl_stream_t stream, void** b, const void* opaque, s
     unsigned char* scratch = static_cast<unsigned char*>(b[2]);
     uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
     const int w = kObsDimM * 2 / 16;  // uint4 per bf16 observation row
-    k_gather_obs_rows<<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
+    k_gather_obs_rows<false><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
                                                                      gathered, n, w);
     ActArgs act{};
     act.mask = static_cast<const uint8_t*>(b[3]);
@@ -1118,6 +1208,54 @@ int32_t brl_policy_act_rows(brl_stream_t stream, void** b, const void* opaque, s
     act.row_index = static_cast<const int32_t*>(b[5]);
     return mlp_forward_impl("brl_policy_act_rows", s, p, gathered, static_cast<const unsigned char*>(b[1]),
                             reinterpret_cast<__nv_bfloat16*>(scratch), static_cast<float*>(b[7]), nullptr, act);
+}
+
+int64_t brl_mlp_pool_stride(void) { return (int64_t)mlp_layout().total; }  // a multiple of 256: every section keeps its TMA alignment
+
+int64_t brl_model_rows_capacity(int64_t n_envs, int64_t n_models) {  // every group rounded up to kGroupRows rows
+    if (n_envs <= 0 || n_models <= 0) return 0;
+    const int64_t groups = n_models < n_envs ? n_models : n_envs;
+    return (n_envs + groups * (kGroupRows - 1)) / kGroupRows * kGroupRows;
+}
+
+int64_t brl_policy_grouped_scratch_bytes(int64_t n_envs, int64_t n_models) {
+    return brl_mlp_rows_scratch_bytes(brl_model_rows_capacity(n_envs, n_models));
+}
+
+// `team_forward_pass.apply` + masked argmax for every listed env with ITS net out of a pool (src/evaluation.py:124-151 for all
+// matches of workspace/eval_selfplay_league.py at once): the rows come grouped by net and padded per group (brl_model_rows),
+// so every kGroupRows-row block runs one net; the weight operands are 3-D tensor maps over the stacked blobs.
+int32_t brl_policy_act_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    BRL_REQUIRE(b[0], "obs_bf16");
+    BRL_REQUIRE(b[1], "pool");
+    BRL_REQUIRE(b[2], "scratch");
+    BRL_REQUIRE(b[4], "action");
+    BRL_REQUIRE(b[5], "rows");
+    BRL_REQUIRE(b[6], "block_model");
+    if (b[3] != nullptr && (reinterpret_cast<uintptr_t>(b[3]) & 1u)) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: mask is misaligned");
+    if (b[7] != nullptr && (reinterpret_cast<uintptr_t>(b[7]) & 7u)) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: logits is misaligned");
+    if (p->k_steps <= 0) return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: k_steps (the pool's model count) must be > 0");
+    if (p->n_envs % kGroupRows != 0)
+        return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: n_envs (padded rows) must be a multiple of %d", kGroupRows);
+    if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: sampling is not supported (argmax only)");
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = p->n_envs;
+    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
+    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
+    const int w = kObsDimM * 2 / 16;
+    k_gather_obs_rows<true><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
+                                                                           gathered, n, w);
+    ActArgs act{};
+    act.mask = static_cast<const uint8_t*>(b[3]);
+    act.action = static_cast<int32_t*>(b[4]);
+    act.row_index = static_cast<const int32_t*>(b[5]);
+    const PoolArgs pool{static_cast<const int32_t*>(b[6]), brl_mlp_pool_stride(), p->k_steps, act};
+    return mlp_forward_impl<true>("brl_policy_act_grouped", s, p, gathered, static_cast<const unsigned char*>(b[1]),
+                                  reinterpret_cast<__nv_bfloat16*>(scratch), static_cast<float*>(b[7]), nullptr, act, &pool);
 }
 
 int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t len) {

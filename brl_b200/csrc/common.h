@@ -47,6 +47,10 @@ inline int device_slot() {
     return dev >= 0 && dev < kMaxDevices ? dev : 0;
 }
 
+// Grouped forward over a pool of nets (brl_model_rows -> brl_policy_act_grouped): each net's rows are padded to this height,
+// the row tile of the fused forward's CTA pairs, so that no tile mixes two nets.
+constexpr int kGroupRows = 256;
+
 // masked categorical over f32 logits[n,38] (brl_algo.cu); shared by brl_categorical and the unfused brl_policy_act path
 int32_t launch_categorical(cudaStream_t stream, const float* logits, const unsigned char* mask, int32_t* action, float* log_prob,
                            int64_t n, int sample, uint64_t seed, int64_t env_offset, uint32_t step, const int32_t* row_index = nullptr,

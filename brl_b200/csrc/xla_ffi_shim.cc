@@ -71,6 +71,9 @@
     X(brl_sl_examples, "iiiiiooooo") \
     X(brl_sl_grad, "iisiioos") \
     X(brl_sl_eval, "iisiios") \
+    X(brl_model_rows, "iiioooo") \
+    X(brl_policy_act_grouped, "iisixiix") \
+    X(brl_match_stats_ranges, "iix") \
     /* end */
 
 namespace {

@@ -483,3 +483,79 @@ def state_fields(state: torch.Tensor) -> dict:
     _call("brl_state_fields", [_ptr(state)] + [_ptr(out[name]) for name, _, _ in _FIELD_SPECS],
               _params(n, stride=state.shape[1]))
     return out
+
+
+# ---- self-play league over a pool of nets (workspace/eval_selfplay_league.py) ----------------------------------------
+def _size_query(name: str, *args) -> int:
+    fn = getattr(_lib.load(), name)
+    fn.restype, fn.argtypes = _lib.C.c_int64, [_lib.C.c_int64] * len(args)
+    return int(fn(*args))
+
+
+def mlp_pool_stride() -> int:
+    """bytes between two nets of a pool blob (a packed blob, padded to keep every section's TMA alignment)"""
+    return _size_query("brl_mlp_pool_stride")
+
+
+def model_rows_capacity(n_envs: int, n_models: int) -> int:
+    """rows `model_rows` may need for n_envs envs over n_models nets (each group padded to 256 rows)"""
+    return _size_query("brl_model_rows_capacity", n_envs, n_models)
+
+
+def policy_grouped_scratch_bytes(n_envs: int, n_models: int) -> int:
+    return _size_query("brl_policy_grouped_scratch_bytes", n_envs, n_models)
+
+
+def mlp_pack_pool(params_list, pack_one) -> torch.Tensor:
+    """Stack the packed blobs of `params_list` as u8[M, mlp_pool_stride()]; `pack_one(params, out)` packs one net into
+    `out` (ForwardPass.pack_into, i.e. mlp_pack(out=...))."""
+    if not params_list:
+        raise _lib.BrlError("mlp_pack_pool: empty pool")
+    dev = next(iter(params_list[0].values()))["w"].device
+    pool = torch.zeros((len(params_list), mlp_pool_stride()), dtype=torch.uint8, device=dev)
+    size = _lib.load().brl_mlp_packed_bytes()
+    for m, params in enumerate(params_list):
+        pack_one(params, pool[m, :size])
+    return pool
+
+
+def model_rows(current_player: torch.Tensor, done: Optional[torch.Tensor], env_models: torch.Tensor, rows: torch.Tensor,
+               counts: torch.Tensor, offsets: torch.Tensor, block_model: torch.Tensor) -> None:
+    """Live envs (done == 0) grouped by the net that acts there: env_models[i, 0] for players 0/1, [i, 1] for players 2/3.
+    Net m's rows are rows[offsets[m] : offsets[m] + counts[m]], padded with -1 to offsets[m + 1]; offsets[M] is the padded
+    row count and block_model the net of each 256-row block.  A live env whose id is outside [0, M) makes offsets[M] = -1:
+    the grouping is invalid, and the caller's read of offsets[M] (which sizes the forward) must raise."""
+    n_models = counts.shape[0]
+    if env_models.dtype != torch.int32 or tuple(env_models.shape) != (current_player.shape[0], 2):
+        raise _lib.BrlError("model_rows: env_models must be int32 [n, 2]")
+    if offsets.shape[0] != n_models + 1 or rows.shape[0] < model_rows_capacity(current_player.shape[0], n_models):
+        raise _lib.BrlError("model_rows: offsets must hold M + 1 entries and rows model_rows_capacity(n, M)")
+    _call("brl_model_rows", [_ptr(current_player), _ptr(done), _ptr(env_models), _ptr(rows), _ptr(counts), _ptr(offsets),
+                             _ptr(block_model)], _params(current_player.shape[0], k_steps=n_models))
+
+
+def policy_act_grouped(obs_bf16: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, mask: Optional[torch.Tensor],
+                       action: torch.Tensor, rows: torch.Tensor, block_model: torch.Tensor,
+                       logits: Optional[torch.Tensor] = None, *, single_bf16: bool = False, tune: int = 0) -> None:
+    """`policy_act_rows` (masked argmax) for the padded, net-grouped `rows` of `model_rows`, net block_model[b] on rows
+    [256 b, 256 b + 256), all nets of `pool` (u8[M, mlp_pool_stride()]) in one forward.  rows / block_model must come from
+    `model_rows` with the same M (device data, not checked here)."""
+    n = rows.shape[0]
+    if n == 0:
+        return
+    if obs_bf16.dtype != torch.bfloat16 or rows.dtype != torch.int32 or block_model.dtype != torch.int32:
+        raise _lib.BrlError("policy_act_grouped needs a bf16 observation and int32 rows / block_model")
+    if pool.dim() != 2 or pool.shape[1] != mlp_pool_stride() or pool.dtype != torch.uint8:
+        raise _lib.BrlError("policy_act_grouped: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    if scratch.numel() < _lib.load().brl_mlp_rows_scratch_bytes(n):
+        raise _lib.BrlError("policy_act_grouped: scratch too small (ops.policy_grouped_scratch_bytes)")
+    _call("brl_policy_act_grouped", [_ptr(obs_bf16), _ptr(pool), _ptr(scratch), _ptr(mask), _ptr(action), _ptr(rows),
+                                     _ptr(block_model), _ptr(logits)],
+          _params(n, k_steps=pool.shape[0], flags=(F_MLP_BF16 if single_bf16 else 0) | tune))
+
+
+def match_stats_ranges(x: torch.Tensor, offsets: torch.Tensor, sums: torch.Tensor) -> None:
+    """sums[p, :4] += match_stats of x[offsets[p]:offsets[p + 1]] for every range p (offsets int64[P + 1], sums f64[P, 8])."""
+    if offsets.dtype != torch.int64 or sums.dtype != torch.float64 or tuple(sums.shape) != (offsets.shape[0] - 1, 8):
+        raise _lib.BrlError("match_stats_ranges: offsets must be int64[P + 1] and sums float64[P, 8]")
+    _call("brl_match_stats_ranges", [_ptr(x), _ptr(offsets), _ptr(sums)], _params(sums.shape[0]))

@@ -59,6 +59,11 @@
  *   brl_sl_examples       make_dataset: replay of a stored auction prefix -> (obs, legal mask, label)   sl.py:87-117
  *   brl_sl_grad           jax.value_and_grad(loss)(params, inputs, targets, legal_actions)             sl.py:169-184,205-206
  *   brl_sl_eval           loss + accuracy + illegal-action probability, no gradient                     sl.py:169-194,288-301
+ *   brl_model_rows        the per-team net choice of every league match: live rows grouped by acting net
+ *                                                      workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
+ *   brl_policy_act_grouped  team{1,2}_forward_pass.apply + masked argmax of every match of a league, one forward over a
+ *                         pool of nets                 workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
+ *   brl_match_stats_ranges  brl_match_stats of every match of a league chunk   src/evaluation.py:199-201
  */
 #ifndef BRL_B200_H
 #define BRL_B200_H
@@ -255,6 +260,38 @@ int32_t brl_policy_act_rows(brl_stream_t, void **buffers, const void *opaque, si
  *          [3] out i32 rows_team2[n]  [4] out i32 counts[2] */
 int32_t brl_team_rows(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- self-play league over a pool of M nets (workspace/eval_selfplay_league.py; each match src/evaluation.py:69-204) ----
+ * All matches of the league run as one batch of envs.  The pool is M packed blobs (brl_mlp_pack) stacked
+ * brl_mlp_pool_stride() bytes apart.  Every live env is forwarded by the net that acts there, with a one-host-read-per-step
+ * loop: brl_model_rows groups the rows by net, the host reads offsets[M] (the padded row count; 0 = every env finished),
+ * brl_policy_act_grouped runs all nets in one forward.  BrlParams.k_steps = M in both. */
+int64_t brl_mlp_pool_stride(void);
+/* rows a grouping of n_envs envs over M nets can need: each non-empty group is padded to 256 rows (one row tile) */
+int64_t brl_model_rows_capacity(int64_t n_envs, int64_t n_models);
+/* k_team_rows generalised (src/evaluation.py:124-151 with a net per env and team): env i is live unless done[i]; its acting
+ * net is env_models[i][0] for players 0/1 and env_models[i][1] for players 2/3.  A live env whose id is outside [0, M) is an
+ * error: offsets[M] comes back as -1 (the host reads offsets[M] anyway to size the forward; the other outputs are then invalid).
+ * buffers: [0] in i8 current_player[n]  [1] in u8 done[n] (NULL -> all live)  [2] in i32 env_models[n,2]
+ *          [3] out i32 rows[brl_model_rows_capacity(n, M)]: net m's live envs at [offsets[m], offsets[m] + counts[m]), then -1
+ *              up to offsets[m + 1]  [4] out i32 counts[M]  [5] out i32 offsets[M + 1] (multiples of 256; offsets[M] = the
+ *              padded row count)  [6] out i32 block_model[capacity / 256]: the net of each 256-row block
+ * An empty batch (n_envs = 0) zeroes counts / offsets when they are given. */
+int32_t brl_model_rows(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_policy_act_rows with the net of each row block taken from the pool (masked argmax only; BRL_F_SAMPLE is an error).
+ * n_envs = the padded row count offsets[M] of brl_model_rows; action and logits of the listed envs are written by env.
+ * buffers: [0] in bf16 obs[total,480]  [1] in pool u8[M, brl_mlp_pool_stride()]  [2] scratch
+ *          (brl_policy_grouped_scratch_bytes(total, M))  [3] in u8 mask[total,38] (NULL -> unmasked)  [4] out i32 action[total]
+ *          [5] in i32 rows[n_envs]  [6] in i32 block_model[n_envs / 256]  [7] out f32 logits[total,38] (NULL ok)
+ * params: n_envs (a multiple of 256), k_steps = M, flags BRL_F_MLP_BF16.
+ * rows / block_model must be brl_model_rows' output for the same M: they are device data and not checked here; a block id
+ * outside [0, M) is undefined behaviour. */
+int64_t brl_policy_grouped_scratch_bytes(int64_t n_envs, int64_t n_models);
+int32_t brl_policy_act_grouped(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_match_stats over P = n_envs contiguous ranges (the matches of a league chunk), each entry exactly what brl_match_stats
+ * gives on that slice.  buffers: [0] in f32 x  [1] in i64 offsets[P + 1] (range p = [offsets[p], offsets[p + 1]))
+ *          [2] inout f64 sums[P, 8] */
+int32_t brl_match_stats_ranges(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -441,6 +478,9 @@ void brl_mlp_forward_xla(brl_stream_t, void **buffers, const char *opaque, size_
 void brl_policy_act_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_policy_act_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_team_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_model_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_policy_act_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_match_stats_ranges_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_loss_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_clip_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_apply_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
