@@ -356,7 +356,6 @@ int32_t brl_gae(brl_stream_t stream, void** b, const void* opaque, size_t len) {
     for (int k = 0; k < 6; ++k)
         if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_gae: buffer '%s' is NULL", names[k]);
     if (p->k_steps <= 0) return fail(BRL_E_OPAQUE, "brl_gae: k_steps (T) must be > 0");
-    if (p->n_envs == 0) return BRL_OK;
     k_gae<<<(unsigned)((p->n_envs + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         static_cast<const uint8_t*>(b[0]), static_cast<const float*>(b[1]), static_cast<const float*>(b[2]),
         static_cast<const float*>(b[3]), static_cast<float*>(b[4]), static_cast<float*>(b[5]), p->k_steps, p->n_envs,
@@ -370,7 +369,6 @@ int32_t brl_categorical(brl_stream_t stream, void** b, const void* opaque, size_
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     if (b[0] == nullptr) return fail(BRL_E_BUFFER, "brl_categorical: buffer 'logits' is NULL");
-    if (p->n_envs == 0) return BRL_OK;
     return launch_categorical((cudaStream_t)stream, static_cast<const float*>(b[0]), static_cast<const uint8_t*>(b[1]),
                               static_cast<int32_t*>(b[2]), static_cast<float*>(b[3]), p->n_envs,
                               (p->flags & BRL_F_SAMPLE) ? 1 : 0, p->seed, p->env_offset, p->step, nullptr);
@@ -389,7 +387,6 @@ int32_t brl_team_rows(brl_stream_t stream, void** b, const void* opaque, size_t 
     BRL_REQUIRE(b[3], "rows_team2");
     BRL_REQUIRE(b[4], "counts");
     if (cudaMemsetAsync(b[4], 0, 2 * sizeof(int32_t), (cudaStream_t)stream) != cudaSuccess) return check_launch("brl_team_rows");
-    if (p->n_envs == 0) return BRL_OK;
     unsigned grid = (unsigned)((p->n_envs + 1023) / 1024);
     k_team_rows<<<grid, 1024, 0, (cudaStream_t)stream>>>(static_cast<const int8_t*>(b[0]), static_cast<const uint8_t*>(b[1]),
                                                          static_cast<int32_t*>(b[2]), static_cast<int32_t*>(b[3]),
@@ -405,7 +402,6 @@ int32_t brl_imp_reward(brl_stream_t stream, void** b, const void* opaque, size_t
     BRL_REQUIRE(b[0], "a_rewards");
     BRL_REQUIRE(b[1], "b_rewards");
     BRL_REQUIRE(b[2], "imp");
-    if (p->n_envs == 0) return BRL_OK;
     k_imp_reward<<<(unsigned)((p->n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         static_cast<const float4*>(b[0]), static_cast<const float4*>(b[1]), static_cast<float4*>(b[2]), p->n_envs);
     return check_launch("brl_imp_reward");
@@ -417,7 +413,6 @@ int32_t brl_match_stats(brl_stream_t stream, void** b, const void* opaque, size_
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     if (b[0] == nullptr || b[1] == nullptr) return fail(BRL_E_BUFFER, "brl_match_stats: NULL buffer");
-    if (p->n_envs == 0) return BRL_OK;
     unsigned grid = (unsigned)((p->n_envs + 255) / 256);
     if (grid > 148u * 4u) grid = 148u * 4u;
     k_match_stats<<<grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const float*>(b[0]), static_cast<double*>(b[1]),
@@ -480,7 +475,6 @@ int32_t brl_gather_reward(brl_stream_t stream, void** b, const void* opaque, siz
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     if (b[0] == nullptr || b[1] == nullptr || b[2] == nullptr) return fail(BRL_E_BUFFER, "brl_gather_reward: NULL buffer");
-    if (p->n_envs == 0) return BRL_OK;
     const bool counting = (p->flags & BRL_F_COUNT_DONE) != 0;
     if (counting && (b[3] == nullptr || b[4] == nullptr || (reinterpret_cast<uintptr_t>(b[4]) & 7u)))
         return fail(BRL_E_BUFFER, "brl_gather_reward: BRL_F_COUNT_DONE needs buffers [3] done and [4] count (8-byte aligned)");

@@ -873,7 +873,6 @@ int32_t brl_make_keys(brl_stream_t stream, void** b, const void* opaque, size_t 
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     BRL_REQUIRE(b[0], "keys");
-    if (p->n_envs == 0) return BRL_OK;
     k_make_keys<<<(unsigned)((p->n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         static_cast<uint64_t*>(b[0]), p->n_envs, p->seed, p->env_offset);
     return check_launch("brl_make_keys");
@@ -1027,7 +1026,6 @@ int32_t brl_legal_mask(brl_stream_t stream, void** b, const void* opaque, size_t
     fill_common(a, p);
     a.state_in = static_cast<const uint4*>(b[0]);
     a.mask = static_cast<uint8_t*>(b[1]);
-    if (a.n == 0) return BRL_OK;
     // 256 * 38 bytes per block is a multiple of 16, so every block's run starts 16-byte aligned when the buffer is
     k_legal_mask<<<(unsigned)((a.n + kMaskEnvsPerBlock - 1) / kMaskEnvsPerBlock), kMaskEnvsPerBlock, 0, (cudaStream_t)stream>>>(
         a.state_in, a.stride, a.mask, a.n, mask_vec_ok(a.mask, a.n, 1));
@@ -1072,7 +1070,6 @@ int32_t brl_state_fields(brl_stream_t stream, void** b, const void* opaque, size
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     BRL_REQUIRE(b[0], "state");
-    if (p->n_envs == 0) return BRL_OK;
     FieldArgs a;
     a.state = static_cast<const uint4*>(b[0]);
     a.deal = static_cast<int32_t*>(b[1]);

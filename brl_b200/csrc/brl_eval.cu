@@ -171,7 +171,6 @@ int32_t brl_eval_act_log(brl_stream_t stream, void** b, const void* opaque, size
     static const char* names[] = {"logits_actor", "logits_opp", "mask", "current_player", "terminated", "action", "acc"};
     for (int k = 0; k < 7; ++k)
         if (b[k] == nullptr && k != 1) return fail(BRL_E_BUFFER, "brl_eval_act_log: buffer '%s' is NULL", names[k]);
-    if (p->n_envs == 0) return BRL_OK;
     ActLogArgs a;
     a.l_actor = static_cast<const float*>(b[0]);
     a.l_opp = static_cast<const float*>(b[1]);
@@ -197,7 +196,6 @@ int32_t brl_eval_summary(brl_stream_t stream, void** b, const void* opaque, size
     for (int k = 0; k < 7; ++k)
         if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_eval_summary: buffer '%s' is NULL", names[k]);
     if (b[15] == nullptr) return fail(BRL_E_BUFFER, "brl_eval_summary: buffer 'sums' is NULL");
-    if (p->n_envs == 0) return BRL_OK;
     SummaryArgs a;
     a.acc = static_cast<const float*>(b[0]);
     a.cum_return = static_cast<const float*>(b[1]);

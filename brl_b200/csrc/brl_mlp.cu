@@ -1,6 +1,6 @@
 // brl_mlp.cu -- the policy/value net of the rollout and evaluation loops on the 5th-gen
 // tensor cores: the "DeepMind" 480 -> 4 x 1024 ReLU -> {38 logits, 1 value} MLP
-// (src/models.py:23-33) as five TMA + tcgen05 GEMM launches.  sm_100a only.
+// (src/models.py:23-33) on TMA + tcgen05 GEMM tiles.  sm_100a only.
 //
 // The reference runs this net in fp32 (haiku default).  A single bf16 product would
 // change near-tie argmax decisions, so the default mode here is a THREE-TERM bf16 split
@@ -10,7 +10,10 @@
 // layer's input is the 0/1 observation, exact in bf16, so it needs only two terms.
 // BRL_F_MLP_BF16 selects the plain single-product mode.
 //
-// One layer = one launch of k_mlp_layer: C[M, N] = act(A[M, K] . Wt[N, K]^T + b).
+// Two forward paths, chosen by batch size (fused_forward): below kPairMinM = 4096 rows, five launches of k_mlp_layer;
+// from 4096 rows on, one persistent launch of k_mlp_fused for the whole net.
+//
+// k_mlp_layer, one layer per launch: C[M, N] = act(A[M, K] . Wt[N, K]^T + b).
 //   Persistent, one CTA per SM; CTA tile 128 (envs) x BN (features), K in blocks of 64 bf16 = one 128-byte
 //   swizzle row; two TMEM accumulators so the epilogue of one tile overlaps the main loop of the next.
 //   warp 0    TMA producer: per K block, bulk-tensor loads of the A / Wt (hi, lo) boxes into a
@@ -19,6 +22,8 @@
 //             accumulate in TMEM); tcgen05.commit hands the stage back / signals the epilogue;
 //   warps 2-5 epilogue: tcgen05.ld the accumulator (thread = one env row), + bias, ReLU,
 //             split into bf16 hi / lo for the next layer (or fp32 logits + value for the head).
+// k_mlp_fused, all five layers in one launch: the same roles on CTA pairs (cta_group::2, 256-row tiles), with every
+//   layer's tiles in one list and per-row-block counters in place of the launch boundaries between layers.
 #include <cuda.h>
 #include <cuda_bf16.h>
 
@@ -398,7 +403,7 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
     if (warp == 1) tmem_dealloc(tmem_acc, kTmemCols);
 }
 
-// ---- one hidden layer on CTA PAIRS (cta_group::2) ------------------------------------------------
+// ---- CTA pairs (cta_group::2): the tiles of k_mlp_fused -----------------------------------------
 // The 1-CTA tiles above are bound by the L2 -> SM operand fill (~64 B/clk/SM against the split mode's
 // 83 B/clk demand at 128 x 128).  A CTA pair (cluster of 2 = the two SMs of a TPC) computes a 256 x BN tile
 // with ONE tcgen05.mma.cta_group::2 stream issued by the leader: each CTA stages its own 128 env rows of A and
@@ -406,7 +411,7 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
 // own 128 x BN block in its own TMEM.  Operand bytes per MMA clock: 42 B/clk/SM at BN = 256.
 //   full[s]        lives in the leader; both CTAs' TMA loads complete_tx on it (cta_group::2, peer bit masked);
 //   empty[s]       one per CTA, released by the leader's multicast tcgen05.commit;
-//   tmem_full[b]   one per CTA, multicast commit;   tmem_empty[b]  in the leader, 8 arrivals (4 epilogue warps x 2).
+//   tmem_full[b]   one per CTA, multicast commit;   tmem_empty[b]  in the leader, 16 arrivals (8 epilogue warps x 2 CTAs).
 constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;  // shared::cluster address of the same offset in the pair's even CTA
 
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -438,134 +443,6 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {  // arrives on `bar`'s offset in BOTH CTAs
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                  ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-
-template <int BN, bool SPLIT_A, bool SPLIT_W>
-struct PairCfg {
-    static constexpr uint32_t kABytes = kBM * kBK * 2, kWBytes = (BN / 2) * kBK * 2;  // per CTA: own A rows, half of Wt
-    static constexpr uint32_t kStageBytes = kABytes * (SPLIT_A ? 2 : 1) + kWBytes * (SPLIT_W ? 2 : 1);
-    static constexpr int kStages = (kSmemBudget / kStageBytes) > 8 ? 8 : (int)(kSmemBudget / kStageBytes);
-    static constexpr uint32_t kSmemBytes = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
-};
-
-template <int BN, bool SPLIT_A, bool SPLIT_W>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMlpThreads, 1)
-k_mlp_layer_pair(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
-                 const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, const LayerArgs a) {
-    using Cfg = PairCfg<BN, SPLIT_A, SPLIT_W>;
-    constexpr int S = Cfg::kStages;
-    constexpr uint32_t kTmemCols = 2 * BN;
-    static_assert(kTmemCols <= 512, "two accumulators must fit tensor memory");
-    extern __shared__ unsigned char smem_dyn[];
-    const uint32_t base = (smem_addr(smem_dyn) + 1023u) & ~1023u;  // same offset in both CTAs of the pair
-    const uint32_t bar_base = base + S * Cfg::kStageBytes;
-    auto full_bar = [&](int s) { return bar_base + 8u * s; };
-    auto empty_bar = [&](int s) { return bar_base + 8u * (S + s); };
-    auto tmem_full_bar = [&](int b) { return bar_base + 8u * (2 * S + b); };
-    auto tmem_empty_bar = [&](int b) { return bar_base + 8u * (2 * S + 2 + b); };
-    const uint32_t store_base = (bar_base + 256u + 1023u) & ~1023u;  // 8 epilogue warps x (hi, lo) x 2 KB store staging
-    __shared__ uint32_t tmem_base_s;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const bool leader = rank == 0;
-    const int n_tiles_n = a.n_tiles_n, n_tiles = a.n_tiles;       // pair tiles: 256 rows x BN columns
-    const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_a_hi) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_w_hi) : "memory");
-        if (SPLIT_A) asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_a_lo) : "memory");
-        if (SPLIT_W) asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_w_lo) : "memory");
-        for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(tmem_full_bar(b), 1); mbar_init(tmem_empty_bar(b), 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    if (warp == 1) {  // the same warp of both CTAs allocates the pair's tensor memory
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&tmem_base_s)), "r"(kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    cluster_sync_all();  // barriers of both CTAs initialised before any remote arrive / multicast commit
-    tc_fence_after();
-    const uint32_t tmem_acc = *reinterpret_cast<volatile uint32_t*>(&tmem_base_s);
-
-    if (warp == 0) {
-        if (lane == 0) {  // ===== TMA producer (both CTAs: own A rows, own half of the Wt rows) =====
-            const uint32_t lead_full0 = full_bar(0) & kPeerBitMask;
-            uint32_t it = 0;
-            for (int tile = pair; tile < n_tiles; tile += n_pairs) {
-                const int m0 = (tile / n_tiles_n) * (2 * kBM) + (int)rank * kBM;
-                const int n0 = (tile % n_tiles_n) * BN + (int)rank * (BN / 2);
-                for (int kb = 0; kb < a.k_blocks; ++kb, ++it) {
-                    const int s = (int)(it % S);
-                    mbar_wait(empty_bar(s), ((it / S) & 1u) ^ 1u);
-                    if (leader) mbar_expect_tx(full_bar(s), 2u * Cfg::kStageBytes);  // both CTAs' bytes land on the leader's barrier
-                    const uint32_t fb = lead_full0 + 8u * s;
-                    uint32_t dst = base + s * Cfg::kStageBytes;
-                    tma_load_2d_pair(dst, &tm_a_hi, fb, kb * kBK, m0);
-                    dst += Cfg::kABytes;
-                    if (SPLIT_A) { tma_load_2d_pair(dst, &tm_a_lo, fb, kb * kBK, m0); dst += Cfg::kABytes; }
-                    tma_load_2d_pair(dst, &tm_w_hi, fb, kb * kBK, n0);
-                    dst += Cfg::kWBytes;
-                    if (SPLIT_W) tma_load_2d_pair(dst, &tm_w_lo, fb, kb * kBK, n0);
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (leader && lane == 0) {  // ===== MMA issuer: the leader drives both SMs' tensor cores =====
-            constexpr uint32_t idesc = umma_idesc_bf16(2 * kBM, BN);
-            uint32_t it = 0, j = 0;
-            for (int tile = pair; tile < n_tiles; tile += n_pairs, ++j) {
-                const uint32_t buf = j & 1u;
-                mbar_wait(tmem_empty_bar(buf), ((j >> 1) & 1u) ^ 1u);  // both CTAs' epilogues have drained this accumulator
-                tc_fence_after();
-                const uint32_t acc = tmem_acc + buf * BN;
-                for (int kb = 0; kb < a.k_blocks; ++kb, ++it) {
-                    const int s = (int)(it % S);
-                    mbar_wait(full_bar(s), (it / S) & 1u);
-                    tc_fence_after();
-                    const uint32_t sa_hi = base + s * Cfg::kStageBytes;
-                    const uint32_t sa_lo = sa_hi + Cfg::kABytes;
-                    const uint32_t sw_hi = sa_hi + Cfg::kABytes * (SPLIT_A ? 2 : 1);
-                    const uint32_t sw_lo = sw_hi + Cfg::kWBytes;
-#pragma unroll
-                    for (int k = 0; k < kBK / kUmmaK; ++k) {
-                        const uint32_t koff = (uint32_t)k * kUmmaK * 2;
-                        const uint64_t da_hi = umma_desc_sw128(sa_hi + koff), dw_hi = umma_desc_sw128(sw_hi + koff);
-                        umma_bf16_pair(acc, da_hi, dw_hi, idesc, (kb | k) != 0);
-                        if (SPLIT_A) umma_bf16_pair(acc, umma_desc_sw128(sa_lo + koff), dw_hi, idesc, 1u);
-                        if (SPLIT_W) umma_bf16_pair(acc, da_hi, umma_desc_sw128(sw_lo + koff), idesc, 1u);
-                    }
-                    umma_commit_pair(empty_bar(s));
-                }
-                umma_commit_pair(tmem_full_bar(buf));
-            }
-        }
-    } else {  // ===== epilogue: warps 2..5 of each CTA drain that CTA's own 128 rows =====
-        const int q = warp & 3;
-        const uint32_t lead_tmem_empty0 = tmem_empty_bar(0) & kPeerBitMask;
-        uint32_t j = 0;
-        for (int tile = pair; tile < n_tiles; tile += n_pairs, ++j) {
-            const int m0 = (tile / n_tiles_n) * (2 * kBM) + (int)rank * kBM, n0 = (tile % n_tiles_n) * BN;
-            const uint32_t buf = j & 1u;
-            mbar_wait(tmem_full_bar(buf), (j >> 1) & 1u);
-            tc_fence_after();
-            const int row = m0 + q * 32 + lane;
-            const uint32_t t_row = tmem_acc + buf * BN + ((uint32_t)(q * 32) << 16);
-            const float* bias = a.bias + n0;
-            epilogue_hidden_row(t_row, BN, bias, row < a.M, a.out_hi + (size_t)row * a.n_total + n0,
-                                a.out_lo ? a.out_lo + (size_t)row * a.n_total + n0 : nullptr);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0)  // remote arrive on the leader's barrier (local for the leader itself)
-                asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(lead_tmem_empty0 + 8u * buf) : "memory");
-        }
-    }
-    tc_fence_before();
-    cluster_sync_all();  // no CTA of the pair may exit (or free tensor memory) while the other still uses its smem / barriers
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(kTmemCols) : "memory");
 }
 
 // ---- the whole forward as ONE persistent launch on CTA pairs ----------------------------------------
@@ -873,50 +750,9 @@ static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, 
     }
     la.n_tiles_n = (n_valid_rows + BN - 1) / BN;
     la.n_tiles = la.n_tiles_n * ((args.M + kBM - 1) / kBM);
-    static int n_sm_dev[kMaxDevices] = {};
-    int& n_sm = n_sm_dev[device_slot()];
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
-    }
+    const int n_sm = sm_count();
     const unsigned grid = (unsigned)(la.n_tiles < n_sm ? la.n_tiles : n_sm);  // persistent: one CTA per SM
     kern<<<grid, kMlpThreads, Cfg::kSmemBytes, s>>>(ta_hi, ta_lo, tw_hi, tw_lo, la);
-    return BRL_OK;
-}
-
-template <int BN, bool SPLIT_A, bool SPLIT_W>
-static int32_t launch_layer_pair(cudaStream_t s, const void* a_hi, const void* a_lo, int k_in, const void* w_hi, const void* w_lo,
-                                 int n_valid_rows, const LayerArgs& args) {
-    using Cfg = PairCfg<BN, SPLIT_A, SPLIT_W>;
-    CUtensorMap ta_hi, ta_lo, tw_hi, tw_lo;
-    bool ok = make_map(&ta_hi, a_hi, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM) &&
-              make_map(&tw_hi, w_hi, (uint64_t)n_valid_rows, (uint64_t)k_in, (uint64_t)k_in, BN / 2);
-    ta_lo = ta_hi;
-    tw_lo = tw_hi;
-    if (ok && SPLIT_A) ok = make_map(&ta_lo, a_lo, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM);
-    if (ok && SPLIT_W) ok = make_map(&tw_lo, w_lo, (uint64_t)n_valid_rows, (uint64_t)k_in, (uint64_t)k_in, BN / 2);
-    if (!ok) return fail(BRL_E_LAUNCH, "brl_mlp_forward: cuTensorMapEncodeTiled failed");
-    auto kern = k_mlp_layer_pair<BN, SPLIT_A, SPLIT_W>;
-    static bool attr_set_dev[kMaxDevices] = {};
-    bool& attr_set = attr_set_dev[device_slot()];
-    if (!attr_set) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
-            return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
-        attr_set = true;
-    }
-    LayerArgs la = args;
-    la.n_tiles_n = n_valid_rows / BN;
-    la.n_tiles = la.n_tiles_n * ((args.M + 2 * kBM - 1) / (2 * kBM));
-    static int n_sm_dev[kMaxDevices] = {};
-    int& n_sm = n_sm_dev[device_slot()];
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
-    }
-    const int n_pairs = la.n_tiles < n_sm / 2 ? la.n_tiles : n_sm / 2;  // persistent: one CTA pair per TPC
-    kern<<<(unsigned)(2 * n_pairs), kMlpThreads, Cfg::kSmemBytes, s>>>(ta_hi, ta_lo, tw_hi, tw_lo, la);
     return BRL_OK;
 }
 
@@ -969,9 +805,7 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
     if (max_pairs == 0) {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
             return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
-        int dev = 0, n_sm = 0;
-        cudaGetDevice(&dev);
-        if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
+        const int n_sm = sm_count();
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = dim3((unsigned)(n_sm & ~1));
         cfg.blockDim = dim3(kFusedThreads);
@@ -1051,7 +885,6 @@ int32_t brl_obs_to_bf16(brl_stream_t stream, void** b, const void* opaque, size_
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     BRL_REQUIRE(b[0], "obs");
     BRL_REQUIRE(b[1], "obs_bf16");
-    if (p->n_envs == 0) return BRL_OK;
     const int64_t n = p->n_envs * kObsDimM;
     const unsigned grid = (unsigned)((n / 8 + 255) / 256);
     if (p->flags & BRL_F_OBS_U8)
@@ -1063,9 +896,16 @@ int32_t brl_obs_to_bf16(brl_stream_t stream, void** b, const void* opaque, size_
 
 }  // extern "C"
 
+// the forward's path: one persistent launch for the whole net once the batch fills the machine, per-layer launches below;
+// BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED force one of them
+static bool fused_forward(const BrlParams* p) {
+    if (p->flags & BRL_F_TUNE_MLP_LAYERS) return false;
+    return (p->flags & BRL_F_TUNE_MLP_FUSED) != 0 || p->n_envs >= kPairMinM;
+}
+
 // forward (+ optional fused categorical) shared by brl_mlp_forward and brl_policy_act.  GROUPED (brl_policy_act_grouped): `blob`
 // is a pool of nets, row block b of the batch runs net pool->block_model[b], and the head epilogue writes action / logits by env
-// (the per-layer head included: no categorical launch).  Its per-layer path has no CTA-pair variant (flags bit 28 is ignored).
+// (the per-layer head included: no categorical launch).
 template <bool GROUPED = false>
 static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams* p, const void* obs, const unsigned char* blob,
                                 __nv_bfloat16* scratch, float* logits, float* value, const ActArgs& act, const PoolArgs* pool = nullptr) {
@@ -1078,10 +918,7 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
     const size_t act_elems = (size_t)M * kHidden;
     __nv_bfloat16* buf_hi[2] = {scratch, scratch + act_elems};
     __nv_bfloat16* buf_lo[2] = {scratch + 2 * act_elems, scratch + 3 * act_elems};
-    // one persistent launch for the whole net once the batch fills the machine; flags bit 30 forces it,
-    // bit 28 forces per-layer CTA-pair launches, bit 29 forbids both (1-CTA tiles)
-    const bool fused = (p->flags & ((1 << 29) | (1 << 28))) ? false : ((p->flags & (1 << 30)) != 0 || M >= kPairMinM);
-    if (fused) {
+    if (fused_forward(p)) {
         uint32_t* ready = reinterpret_cast<uint32_t*>(scratch + 4 * act_elems);
         rc = split ? launch_fused<true, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
                    : launch_fused<false, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
@@ -1105,24 +942,10 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
             a.out_hi = buf_hi[l & 1];
             a.out_lo = split ? buf_lo[l & 1] : nullptr;
             // 128 x 256 tiles move fewer operand bytes per MMA (the L2 -> SM fill rate, ~64 B/clk, is what bounds
-            // these 1-CTA tiles): measured faster for the single-product mode and for large batches
-            // (scripts/exp_mlp_ab.py); flags bit 26 / 27 force wide / narrow
-            const bool wide = (p->flags & (1 << 27)) ? false : ((p->flags & (1 << 26)) != 0 || !split || M >= 32768);
-            const bool pair = !GROUPED && (p->flags & (1 << 28)) != 0;
-            if (pair) {
-                if (l == 0) rc = split ? launch_layer_pair<256, false, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                                       : launch_layer_pair<256, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
-                else rc = split ? launch_layer_pair<256, true, true>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a)
-                                : launch_layer_pair<256, false, false>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a);
-            } else if (wide) {
-                if (l == 0) rc = split ? launch_layer<256, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
-                                       : launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-                else rc = split ? launch_layer<256, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
-                                : launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            } else if (l == 0) rc = split ? launch_layer<128, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
-                                   : launch_layer<128, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            else rc = split ? launch_layer<128, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool)
-                            : launch_layer<128, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            // these 1-CTA tiles): measured faster for the single-product mode; the split mode runs 128 x 128 tiles
+            if (!split) rc = launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else if (l == 0) rc = launch_layer<128, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else rc = launch_layer<128, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
             in_hi = a.out_hi;
             in_lo = a.out_lo;
         } else {
@@ -1140,6 +963,27 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
                               act.row_index ? logits : nullptr);
 }
 
+// brl_policy_act_rows / brl_policy_act_grouped, whose buffers share the slots [0] obs, [1] net or pool, [2] scratch, [3] mask,
+// [4] action, [5] rows, [7] logits: gather the listed rows' observations (one 960-byte bf16 row per thread group) behind the
+// forward's scratch, run the forward on the compact batch, and let the head epilogue read mask[env] and write action[env] /
+// log_prob[env] / logits[env].  GROUPED: row -1 (a group's padding) gathers zeros; block_model = the net of each row block.
+template <bool GROUPED>
+static int32_t policy_act_listed(const char* who, cudaStream_t s, void** b, const BrlParams* p, ActArgs act,
+                                 const int32_t* block_model = nullptr) {
+    const int64_t n = p->n_envs;
+    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
+    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
+    const int w = kObsDimM * 2 / 16;  // uint4 per bf16 observation row
+    k_gather_obs_rows<GROUPED><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]),
+                                                                              static_cast<const int32_t*>(b[5]), gathered, n, w);
+    act.mask = static_cast<const uint8_t*>(b[3]);
+    act.action = static_cast<int32_t*>(b[4]);
+    act.row_index = static_cast<const int32_t*>(b[5]);
+    const PoolArgs pool{block_model, brl_mlp_pool_stride(), p->k_steps, act};
+    return mlp_forward_impl<GROUPED>(who, s, p, gathered, static_cast<const unsigned char*>(b[1]), reinterpret_cast<__nv_bfloat16*>(scratch),
+                                     static_cast<float*>(b[7]), nullptr, act, GROUPED ? &pool : nullptr);
+}
+
 extern "C" {
 
 int32_t brl_mlp_forward(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -1152,7 +996,6 @@ int32_t brl_mlp_forward(brl_stream_t stream, void** b, const void* opaque, size_
     BRL_REQUIRE(b[2], "scratch");
     BRL_REQUIRE(b[3], "logits");
     BRL_REQUIRE(b[4], "value");
-    if (p->n_envs == 0) return BRL_OK;
     return mlp_forward_impl("brl_mlp_forward", (cudaStream_t)stream, p, b[0], static_cast<const unsigned char*>(b[1]),
                             static_cast<__nv_bfloat16*>(b[2]), static_cast<float*>(b[3]), static_cast<float*>(b[4]), ActArgs{});
 }
@@ -1173,8 +1016,7 @@ int64_t brl_mlp_rows_scratch_bytes(int64_t n_rows) {  // brl_mlp_scratch_bytes +
 }
 
 // `team1_forward_pass.apply` + masked Categorical on the LISTED envs only (src/evaluation.py:124-151 without running
-// either net on envs it does not decide): gather the rows' observations (one 960-byte bf16 row per thread group), run
-// the forward on the compact batch, and let the head epilogue read mask[env] and write action[env] / log_prob[env].
+// either net on envs it does not decide).
 int32_t brl_policy_act_rows(brl_stream_t stream, void** b, const void* opaque, size_t len) {
     int32_t rc;
     const BrlParams* p = get_params(opaque, len, &rc);
@@ -1185,29 +1027,15 @@ int32_t brl_policy_act_rows(brl_stream_t stream, void** b, const void* opaque, s
     BRL_REQUIRE(b[2], "scratch");
     BRL_REQUIRE(b[4], "action");
     BRL_REQUIRE(b[5], "row_index");
-    if ((reinterpret_cast<uintptr_t>(b[0]) | reinterpret_cast<uintptr_t>(b[2])) & 15u)
-        return fail(BRL_E_BUFFER, "brl_policy_act_rows: obs / scratch must be 16-byte aligned");
     if (b[3] != nullptr && (reinterpret_cast<uintptr_t>(b[3]) & 1u)) return fail(BRL_E_BUFFER, "brl_policy_act_rows: mask is misaligned");
     if (b[7] != nullptr && (reinterpret_cast<uintptr_t>(b[7]) & 7u)) return fail(BRL_E_BUFFER, "brl_policy_act_rows: logits is misaligned");
-    if (p->n_envs == 0) return BRL_OK;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t n = p->n_envs;
-    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
-    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
-    const int w = kObsDimM * 2 / 16;  // uint4 per bf16 observation row
-    k_gather_obs_rows<false><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
-                                                                     gathered, n, w);
     ActArgs act{};
-    act.mask = static_cast<const uint8_t*>(b[3]);
-    act.action = static_cast<int32_t*>(b[4]);
     act.log_prob = static_cast<float*>(b[6]);
     act.seed = p->seed;
     act.env_offset = p->env_offset;
     act.step = p->step;
     act.sample = (p->flags & BRL_F_SAMPLE) ? 1 : 0;
-    act.row_index = static_cast<const int32_t*>(b[5]);
-    return mlp_forward_impl("brl_policy_act_rows", s, p, gathered, static_cast<const unsigned char*>(b[1]),
-                            reinterpret_cast<__nv_bfloat16*>(scratch), static_cast<float*>(b[7]), nullptr, act);
+    return policy_act_listed<false>("brl_policy_act_rows", (cudaStream_t)stream, b, p, act);
 }
 
 int64_t brl_mlp_pool_stride(void) { return (int64_t)mlp_layout().total; }  // a multiple of 256: every section keeps its TMA alignment
@@ -1242,20 +1070,7 @@ int32_t brl_policy_act_grouped(brl_stream_t stream, void** b, const void* opaque
     if (p->n_envs % kGroupRows != 0)
         return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: n_envs (padded rows) must be a multiple of %d", kGroupRows);
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: sampling is not supported (argmax only)");
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t n = p->n_envs;
-    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
-    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
-    const int w = kObsDimM * 2 / 16;
-    k_gather_obs_rows<true><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
-                                                                           gathered, n, w);
-    ActArgs act{};
-    act.mask = static_cast<const uint8_t*>(b[3]);
-    act.action = static_cast<int32_t*>(b[4]);
-    act.row_index = static_cast<const int32_t*>(b[5]);
-    const PoolArgs pool{static_cast<const int32_t*>(b[6]), brl_mlp_pool_stride(), p->k_steps, act};
-    return mlp_forward_impl<true>("brl_policy_act_grouped", s, p, gathered, static_cast<const unsigned char*>(b[1]),
-                                  reinterpret_cast<__nv_bfloat16*>(scratch), static_cast<float*>(b[7]), nullptr, act, &pool);
+    return policy_act_listed<true>("brl_policy_act_grouped", (cudaStream_t)stream, b, p, ActArgs{}, static_cast<const int32_t*>(b[6]));
 }
 
 int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -1270,7 +1085,6 @@ int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t
     for (int k : {3, 5, 6, 7})
         if (b[k] != nullptr && (reinterpret_cast<uintptr_t>(b[k]) & (k == 3 ? 1u : 7u)) != 0)
             return fail(BRL_E_BUFFER, "brl_policy_act: buffer %d is misaligned", k);
-    if (p->n_envs == 0) return BRL_OK;
     ActArgs act{};
     act.mask = static_cast<const uint8_t*>(b[3]);
     act.action = static_cast<int32_t*>(b[4]);
@@ -1282,7 +1096,9 @@ int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t
     if (p->flags & BRL_F_SEED_SALT) {
         act.seed_salt = static_cast<const uint64_t*>(b[8]);
         if (act.seed_salt == nullptr || (reinterpret_cast<uintptr_t>(b[8]) & 7u)) return fail(BRL_E_BUFFER, "brl_policy_act: BRL_F_SEED_SALT needs an 8-byte aligned buffer [8]");
-        if (p->n_envs < kPairMinM) return fail(BRL_E_OPAQUE, "brl_policy_act: BRL_F_SEED_SALT is supported by the fused launch only (n_envs >= %d)", kPairMinM);
+        if (!fused_forward(p))
+            return fail(BRL_E_OPAQUE, "brl_policy_act: BRL_F_SEED_SALT is supported by the fused launch only (n_envs >= %d, no BRL_F_TUNE_MLP_LAYERS)",
+                        kPairMinM);
     }
     return mlp_forward_impl("brl_policy_act", (cudaStream_t)stream, p, b[0], static_cast<const unsigned char*>(b[1]),
                             static_cast<__nv_bfloat16*>(b[2]), static_cast<float*>(b[7]), static_cast<float*>(b[6]), act);

@@ -709,15 +709,14 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
     fa.nmb = nmb;
     fa.ready = ready;
     fa.trace = trace;
-    static int n_sm_dev[kMaxDevices] = {};
-    int& n_sm = n_sm_dev[device_slot()];
-    if (n_sm == 0) {
+    static bool attr_set_dev[kMaxDevices] = {};
+    bool& attr_set = attr_set_dev[device_slot()];
+    if (!attr_set) {
         if (cudaFuncSetAttribute(k_train_fused<kFBN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
             return fail(BRL_E_LAUNCH, "%s: cannot reserve %u bytes of shared memory", what, Cfg::kSmemBytes);
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
+        attr_set = true;
     }
+    const int n_sm = sm_count();
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)(tiles < n_sm ? tiles : n_sm));  // one CTA per SM: all of them co-resident
     cfg.blockDim = dim3(kMlpThreads);

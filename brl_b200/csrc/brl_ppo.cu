@@ -480,7 +480,6 @@ int32_t brl_gather_rows(brl_stream_t stream, void** b, const void* opaque, size_
     const int64_t B = p->n_envs;
     const int row_bytes = p->k_steps;  // bytes per row
     if (row_bytes <= 0) return fail(BRL_E_OPAQUE, "brl_gather_rows: k_steps (row bytes) must be > 0");
-    if (B == 0) return BRL_OK;
     cudaStream_t s = (cudaStream_t)stream;
     if (row_bytes % 16 == 0) {
         const int w = row_bytes / 16;

@@ -47,6 +47,18 @@ inline int device_slot() {
     return dev >= 0 && dev < kMaxDevices ? dev : 0;
 }
 
+// SM count of the current device, which sizes the persistent grids (148 on a B200 if the query fails)
+inline int sm_count() {
+    static int n_sm_dev[kMaxDevices] = {};
+    int& n_sm = n_sm_dev[device_slot()];
+    if (n_sm == 0) {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm <= 0) n_sm = 148;
+    }
+    return n_sm;
+}
+
 // Grouped forward over a pool of nets (brl_model_rows -> brl_policy_act_grouped): each net's rows are padded to this height,
 // the row tile of the fused forward's CTA pairs, so that no tile mixes two nets.
 constexpr int kGroupRows = 256;

@@ -111,6 +111,10 @@ typedef struct CUstream_st *brl_stream_t; /* == cudaStream_t */
 #define BRL_F_TUNE_WPB8 ((3 << 18) | (1 << 26))
 #define BRL_F_TUNE_CLASSIC_ROLLOUT (1 << 20)     /* tile-per-warp rollout kernel instead of the warp-specialised one */
 #define BRL_F_TUNE_WRITERS(n) ((n) << 21)       /* writer warps (1..7) of the warp-specialised rollout; EPW bits = its envs per block */
+/* the policy forward's path (brl_mlp_forward, brl_policy_act*), chosen by default by batch size: per-layer launches below
+ * 4096 rows, one fused launch from 4096 on.  These bits share none with the env tuning bits above. */
+#define BRL_F_TUNE_MLP_LAYERS (1 << 29)  /* per-layer launches at any size (BRL_F_SEED_SALT is then an error) */
+#define BRL_F_TUNE_MLP_FUSED (1 << 30)   /* the fused launch at any size (ignored with BRL_F_TUNE_MLP_LAYERS) */
 
 /* errors */
 #define BRL_OK 0

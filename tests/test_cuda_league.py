@@ -13,7 +13,7 @@ from tests.test_cuda_xla import _call_xla
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-FORCE_FUSED, FORCE_LAYERS = 1 << 30, 1 << 29
+FORCE_FUSED, FORCE_LAYERS = 1 << 30, 1 << 29  # BRL_F_TUNE_MLP_FUSED, BRL_F_TUNE_MLP_LAYERS (include/brl_b200.h)
 
 
 def _obs_and_mask(n, seed=11, steps=9):

@@ -12,6 +12,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
+FORCE_LAYERS = 1 << 29  # BRL_F_TUNE_MLP_LAYERS (include/brl_b200.h)
 
 
 def _real_obs(n, steps=9, seed=11):
@@ -132,6 +133,20 @@ def test_policy_act_equals_forward_then_categorical(n, sample):
         a3 = torch.full_like(a_ref, -7)
         ops.policy_act(x, blob, scratch, m, a3, sample=sample, seed=99, env_offset=1000)
         assert torch.equal(a3, a_ref)
+
+
+@pytest.mark.parametrize("n,tune", [(100, 0), (4096, FORCE_LAYERS)])
+def test_seed_salt_is_refused_off_the_fused_launch(n, tune):
+    """BRL_F_SEED_SALT is read by the fused launch only: a salted call that runs on the per-layer launches, by its size or
+    forced there, is an error (BRL_E_OPAQUE) rather than a sample drawn with the unsalted seed"""
+    from brl_b200 import _lib, ops
+    obs = torch.zeros((n, 480), dtype=torch.bfloat16, device=DEV)
+    blob = torch.zeros(_lib.load().brl_mlp_packed_bytes(), dtype=torch.uint8, device=DEV)
+    action = torch.full((n,), -7, dtype=torch.int32, device=DEV)
+    salt = torch.zeros(1, dtype=torch.int64, device=DEV)
+    with pytest.raises(_lib.BrlError, match=r"\(-1\).*SEED_SALT"):
+        ops.policy_act(obs, blob, ops.mlp_scratch(n, DEV), None, action, sample=True, tune=tune, seed_salt=salt)
+    assert bool((action == -7).all())
 
 
 def test_product_forward_has_no_library_back_end():
