@@ -267,8 +267,17 @@ struct GroupedLayerArgs : LayerArgs {
     int64_t bias_stride;
     ActArgs act;
 };
-template <bool GROUPED>
-using LayerArgsT = std::conditional_t<GROUPED, GroupedLayerArgs, LayerArgs>;
+// DEVCOUNT (brl_duplicate_match's device loop): the grouped forward's row count is read from device memory; the launch and
+// its tensor maps are sized for the grouping's capacity, and the row blocks past the count exit at once
+struct DevLayerArgs : GroupedLayerArgs {
+    const int32_t* n_rows;  // padded row count (brl_model_rows' offsets[M])
+};
+template <bool GROUPED, bool DEVCOUNT = false>
+using LayerArgsT = std::conditional_t<DEVCOUNT, DevLayerArgs, std::conditional_t<GROUPED, GroupedLayerArgs, LayerArgs>>;
+__device__ __forceinline__ int layer_rows(const LayerArgs& a) { return a.M; }
+__device__ __forceinline__ int layer_rows(const DevLayerArgs& a) { return *a.n_rows; }
+__device__ __forceinline__ int layer_tiles(const LayerArgs& a) { return a.n_tiles; }
+__device__ __forceinline__ int layer_tiles(const DevLayerArgs& a) { return a.n_tiles_n * ((*a.n_rows + kBM - 1) / kBM); }
 
 template <int BN, bool SPLIT_A, bool SPLIT_W>
 struct LayerCfg {
@@ -278,10 +287,11 @@ struct LayerCfg {
     static constexpr uint32_t kSmemBytes = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
 __global__ void __launch_bounds__(kMlpThreads, 1)
 k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
-            const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, const LayerArgsT<GROUPED> a) {
+            const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
+            const LayerArgsT<GROUPED, DEVCOUNT> a) {
     // PERSISTENT: one CTA per SM walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... (n-tile fastest, so the
     // CTAs running together share A row-blocks in L2).  The smem stage ring runs straight across tile
     // boundaries and the accumulator is double-buffered in TMEM, so the epilogue of tile j overlaps the
@@ -299,7 +309,7 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
     __shared__ uint32_t tmem_base_s;  // written by tcgen05.alloc
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_tiles_n = a.n_tiles_n, n_tiles = a.n_tiles;
+    const int n_tiles_n = a.n_tiles_n, n_tiles = layer_tiles(a);
 
     if (warp == 0 && lane == 0) {
         asm volatile("prefetch.tensormap [%0];" ::"l"(&tm_a_hi) : "memory");
@@ -374,7 +384,7 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
             }
         }
     } else {  // ===== epilogue: warps 2..5, TMEM lane quarter = warp % 4 =====
-        const int q = warp & 3;
+        const int q = warp & 3, M = layer_rows(a);
         uint32_t j = 0;
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++j) {
             const int m0 = (tile / n_tiles_n) * kBM, n0 = (tile % n_tiles_n) * BN;
@@ -386,12 +396,12 @@ k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__
             const float* bias = a.bias + n0;
             if constexpr (GROUPED) bias += (size_t)a.block_model[m0 / kGroupRows] * a.bias_stride;
             if constexpr (!HEAD)
-                epilogue_hidden_row(t_row, BN, bias, row < a.M, a.out_hi + (size_t)row * a.n_total + n0,
+                epilogue_hidden_row(t_row, BN, bias, row < M, a.out_hi + (size_t)row * a.n_total + n0,
                                     a.out_lo ? a.out_lo + (size_t)row * a.n_total + n0 : nullptr);
             else if constexpr (GROUPED)  // padding rows of a group (row_index -1) are computed and dropped
-                epilogue_head_act_row(t_row, bias, row < a.M && a.act.row_index[row] >= 0, row, a.logits, nullptr, a.act);
+                epilogue_head_act_row(t_row, bias, row < M && a.act.row_index[row] >= 0, row, a.logits, nullptr, a.act);
             else
-                epilogue_head_row(t_row, bias, row < a.M, a.logits + (size_t)row * 38, a.value + row);
+                epilogue_head_row(t_row, bias, row < M, a.logits + (size_t)row * 38, a.value + row);
             // all of this warp's tcgen05.ld have completed (wait::ld): hand the accumulator back
             tc_fence_before();
             __syncwarp();
@@ -470,8 +480,11 @@ struct GroupedFusedArgs : FusedArgs {  // grouped forward (see GroupedLayerArgs)
     const int32_t* block_model;  // model of each kGroupRows-row block (= the CTA-pair tile height)
     int64_t bias_stride;         // floats between two nets' biases in the pool
 };
-template <bool GROUPED>
-using FusedArgsT = std::conditional_t<GROUPED, GroupedFusedArgs, FusedArgs>;
+struct DevFusedArgs : GroupedFusedArgs {  // DEVCOUNT (see DevLayerArgs): M, nmb and the tile list follow *n_rows
+    const int32_t* n_rows;
+};
+template <bool GROUPED, bool DEVCOUNT = false>
+using FusedArgsT = std::conditional_t<DEVCOUNT, DevFusedArgs, std::conditional_t<GROUPED, GroupedFusedArgs, FusedArgs>>;
 
 constexpr int kFusedBN = 256, kFusedTilesN = kHidden / kFusedBN;
 // Epilogue warps of the fused forward: TWO per TMEM lane quadrant, each draining half of the tile's 256 columns.  One
@@ -530,8 +543,20 @@ __device__ __forceinline__ const float* fused_bias(const GroupedFusedArgs& a, in
 __device__ __forceinline__ bool fused_row_ok(const FusedArgs& a, int row) { return row < a.M; }
 __device__ __forceinline__ bool fused_row_ok(const GroupedFusedArgs& a, int row) { return row < a.M && a.act.row_index[row] >= 0; }
 
-template <bool SPLIT, bool GROUPED = false>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_mlp_fused(const __grid_constant__ FusedArgsT<GROUPED> a) {
+// the launch's shape -- rows, 256-row blocks, tiles per hidden layer, tiles -- from the parameters, or (DEVCOUNT) from *n_rows
+__device__ __forceinline__ int fused_rows(const FusedArgs& a) { return a.M; }
+__device__ __forceinline__ int fused_rows(const DevFusedArgs& a) { return *a.n_rows; }
+__device__ __forceinline__ int fused_nmb(const FusedArgs& a) { return a.nmb; }
+__device__ __forceinline__ int fused_nmb(const DevFusedArgs& a) { return (*a.n_rows + 2 * kBM - 1) / (2 * kBM); }
+__device__ __forceinline__ int fused_tiles_per_layer(const FusedArgs& a) { return a.tiles_per_layer; }
+__device__ __forceinline__ int fused_tiles_per_layer(const DevFusedArgs& a) { return fused_nmb(a) * kFusedTilesN; }
+__device__ __forceinline__ int fused_n_tiles(const FusedArgs& a) { return a.n_tiles; }
+__device__ __forceinline__ int fused_n_tiles(const DevFusedArgs& a) { return fused_nmb(a) * (4 * kFusedTilesN + 1); }
+__device__ __forceinline__ bool fused_row_ok(const DevFusedArgs& a, int row) { return row < *a.n_rows && a.act.row_index[row] >= 0; }
+
+template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1)
+k_mlp_fused(const __grid_constant__ FusedArgsT<GROUPED, DEVCOUNT> a) {
     using Cfg = FusedCfg<SPLIT>;
     constexpr int S = Cfg::kStages;
     constexpr uint32_t kTmemCols = 2 * kFusedBN;
@@ -549,7 +574,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
     const uint32_t rank = cluster_ctarank();
     const bool leader = rank == 0;
     const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-    const int n_tiles = a.n_tiles, tpl = a.tiles_per_layer;
+    const int n_tiles = fused_n_tiles(a), tpl = fused_tiles_per_layer(a);
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < S; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
@@ -584,7 +609,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
                 const CUtensorMap* mw_lo = &a.w_lo[f.layer];
                 BRL_MLP_STAMP(tile, 0);
                 if (f.layer > 0) {  // the previous layer's rows [m0, m0 + 128) must be complete (all 4 n-tiles)
-                    const uint32_t* flag = a.ready + (size_t)(f.layer - 1) * 2 * a.nmb + 2 * f.mb + rank;
+                    const uint32_t* flag = a.ready + (size_t)(f.layer - 1) * 2 * fused_nmb(a) + 2 * f.mb + rank;
                     uint32_t v = 0;
                     for (uint32_t spin = 0;; ++spin) {
                         asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
@@ -674,7 +699,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
                                         m0 + q * 32);
                 } else {
                     __nv_bfloat16* oh = a.out_hi[f.layer];
-                    epilogue_hidden_row(t_row + (uint32_t)(half * kHalfCols), kHalfCols, fused_bias(a, f.layer, f.mb) + n0, row < a.M,
+                    epilogue_hidden_row(t_row + (uint32_t)(half * kHalfCols), kHalfCols, fused_bias(a, f.layer, f.mb) + n0, row < fused_rows(a),
                                         oh + (size_t)row * kHidden + n0, nullptr);
                 }
             } else if (half == 0) {  // the 64-column head tile: one warp per quadrant
@@ -690,7 +715,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1) k_
                         asm volatile("fence.proxy.async;" ::: "memory");
                     }
                     __threadfence();  // cumulative: the warp's rows are visible GPU-wide before the count below
-                    atomicAdd(a.ready + (size_t)f.layer * 2 * a.nmb + 2 * f.mb + rank, 1u);
+                    atomicAdd(a.ready + (size_t)f.layer * 2 * fused_nmb(a) + 2 * f.mb + rank, 1u);
                 }
 #ifdef BRL_MLP_TRACE
                 if (warp == 2 && leader && tile < 1024) { g_mlp_trace[tile][6] = mlp_now(); g_mlp_trace[tile][7] = (unsigned long long)pair; }
@@ -710,6 +735,7 @@ struct PoolArgs {
     int64_t stride;
     int n_models;
     ActArgs act;  // the per-layer head's masked argmax (the fused head takes launch_fused's `act`)
+    const int32_t* n_rows;  // DEVCOUNT: the padded row count in device memory (the launch is sized for M = the capacity)
 };
 
 // weight operand of layer-tile loads: one net's [n_rows, k_in] bf16 matrix, or the pool's {k_in, n_rows, model} stack of them
@@ -721,7 +747,23 @@ static bool make_w_map(CUtensorMap* m, const void* w, uint64_t n_rows, uint64_t 
     return make_map_nd(m, w, 3, dims, strides, box);
 }
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
+// the kernel's shared-memory attribute, set once per device (idempotent, a race only repeats the call); also called ahead of a
+// stream capture (brl_duplicate_match) so that no attribute call falls inside one
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
+static int32_t layer_attr() {
+    using Cfg = LayerCfg<BN, SPLIT_A, SPLIT_W>;
+    static bool attr_set_dev[kMaxDevices] = {};
+    bool& attr_set = attr_set_dev[device_slot()];
+    if (!attr_set) {
+        if (cudaFuncSetAttribute(k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)Cfg::kSmemBytes) != cudaSuccess)
+            return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
+        attr_set = true;
+    }
+    return BRL_OK;
+}
+
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
 static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, int k_in, const void* w_hi, const void* w_lo,
                             int n_valid_rows, const LayerArgs& args, const PoolArgs* pool = nullptr) {
     using Cfg = LayerCfg<BN, SPLIT_A, SPLIT_W>;
@@ -733,21 +775,16 @@ static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, 
     if (ok && SPLIT_A) ok = make_map(&ta_lo, a_lo, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM);
     if (ok && SPLIT_W) ok = make_w_map<GROUPED>(&tw_lo, w_lo, (uint64_t)n_valid_rows, (uint64_t)k_in, BN, pool);
     if (!ok) return fail(BRL_E_LAUNCH, "brl_mlp_forward: cuTensorMapEncodeTiled failed");
-    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED>;
-    static bool attr_set_dev[kMaxDevices] = {};  // per device; idempotent, a race only repeats the call
-    bool& attr_set = attr_set_dev[device_slot()];
-    if (!attr_set) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
-            return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
-        attr_set = true;
-    }
-    LayerArgsT<GROUPED> la{};
+    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>;
+    if (int32_t rc = layer_attr<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>()) return rc;
+    LayerArgsT<GROUPED, DEVCOUNT> la{};
     static_cast<LayerArgs&>(la) = args;
     if constexpr (GROUPED) {
         la.block_model = pool->block_model;
         la.bias_stride = pool->stride / (int64_t)sizeof(float);
         la.act = pool->act;
     }
+    if constexpr (DEVCOUNT) la.n_rows = pool->n_rows;
     la.n_tiles_n = (n_valid_rows + BN - 1) / BN;
     la.n_tiles = la.n_tiles_n * ((args.M + kBM - 1) / kBM);
     const int n_sm = sm_count();
@@ -759,12 +796,47 @@ static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, 
 // counters of the fused forward live behind the four activation buffers of the scratch
 static inline size_t fused_ready_bytes(int64_t n_envs) { return (size_t)(4 * 2 * ((n_envs + 2 * kBM - 1) / (2 * kBM))) * sizeof(uint32_t); }
 
-template <bool SPLIT, bool GROUPED = false>
+// co-resident CTA pairs of the fused kernel (the dependency waits need every launched pair to be running), with its shared-memory
+// attribute set on the first call per device; also called ahead of a stream capture (brl_duplicate_match).  0 = failure.
+template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
+static int fused_pairs() {
+    using Cfg = FusedCfg<SPLIT>;
+    auto kern = k_mlp_fused<SPLIT, GROUPED, DEVCOUNT>;
+    static int max_pairs_dev[kMaxDevices] = {};
+    int& max_pairs = max_pairs_dev[device_slot()];
+    if (max_pairs == 0) {
+        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess) {
+            fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
+            return 0;
+        }
+        const int n_sm = sm_count();
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3((unsigned)(n_sm & ~1));
+        cfg.blockDim = dim3(kFusedThreads);
+        cfg.dynamicSmemBytes = Cfg::kSmemBytes;
+        cudaLaunchAttribute at{};
+        at.id = cudaLaunchAttributeClusterDimension;
+        at.val.clusterDim.x = 2;
+        at.val.clusterDim.y = 1;
+        at.val.clusterDim.z = 1;
+        cfg.attrs = &at;
+        cfg.numAttrs = 1;
+        int n_clusters = 0;
+        if (cudaOccupancyMaxActiveClusters(&n_clusters, kern, &cfg) != cudaSuccess || n_clusters <= 0) {
+            cudaGetLastError();
+            n_clusters = n_sm / 2;
+        }
+        max_pairs = n_clusters < n_sm / 2 ? n_clusters : n_sm / 2;
+    }
+    return max_pairs;
+}
+
+template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
 static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char* blob, const MlpLayout& L, __nv_bfloat16* const buf_hi[2],
                             __nv_bfloat16* const buf_lo[2], uint32_t* ready, float* logits, float* value, int M, const ActArgs& act,
                             const PoolArgs* pool = nullptr) {
     using Cfg = FusedCfg<SPLIT>;
-    FusedArgsT<GROUPED> fa{};
+    FusedArgsT<GROUPED, DEVCOUNT> fa{};
     bool ok = true;
     for (int l = 0; l < 5 && ok; ++l) {
         const void* a_hi = l == 0 ? obs : (const void*)buf_hi[(l - 1) & 1];
@@ -795,35 +867,14 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
         fa.block_model = pool->block_model;
         fa.bias_stride = pool->stride / (int64_t)sizeof(float);
     }
+    if constexpr (DEVCOUNT) fa.n_rows = pool->n_rows;
     fa.M = M;
     fa.nmb = (M + 2 * kBM - 1) / (2 * kBM);
     fa.tiles_per_layer = fa.nmb * kFusedTilesN;
     fa.n_tiles = 4 * fa.tiles_per_layer + fa.nmb;
-    auto kern = k_mlp_fused<SPLIT, GROUPED>;
-    static int max_pairs_dev[kMaxDevices] = {};  // co-resident CTA pairs: the dependency waits need every launched pair to be running
-    int& max_pairs = max_pairs_dev[device_slot()];
-    if (max_pairs == 0) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
-            return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
-        const int n_sm = sm_count();
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(n_sm & ~1));
-        cfg.blockDim = dim3(kFusedThreads);
-        cfg.dynamicSmemBytes = Cfg::kSmemBytes;
-        cudaLaunchAttribute at{};
-        at.id = cudaLaunchAttributeClusterDimension;
-        at.val.clusterDim.x = 2;
-        at.val.clusterDim.y = 1;
-        at.val.clusterDim.z = 1;
-        cfg.attrs = &at;
-        cfg.numAttrs = 1;
-        int n_clusters = 0;
-        if (cudaOccupancyMaxActiveClusters(&n_clusters, kern, &cfg) != cudaSuccess || n_clusters <= 0) {
-            cudaGetLastError();
-            n_clusters = n_sm / 2;
-        }
-        max_pairs = n_clusters < n_sm / 2 ? n_clusters : n_sm / 2;
-    }
+    auto kern = k_mlp_fused<SPLIT, GROUPED, DEVCOUNT>;
+    const int max_pairs = fused_pairs<SPLIT, GROUPED, DEVCOUNT>();
+    if (max_pairs == 0) return BRL_E_LAUNCH;
     if (cudaMemsetAsync(ready, 0, fused_ready_bytes(M), s) != cudaSuccess) return check_launch("brl_mlp_forward (memset)");
     const int n_pairs = fa.n_tiles < max_pairs ? fa.n_tiles : max_pairs;
     kern<<<(unsigned)(2 * n_pairs), kFusedThreads, Cfg::kSmemBytes, s>>>(fa);
@@ -844,6 +895,18 @@ __global__ void __launch_bounds__(256) k_gather_obs_rows(const uint4* __restrict
     } else {
         dst[i] = src[(int64_t)index[r] * w + c];
     }
+}
+
+// the grouped gather of brl_duplicate_match's device loop: launched for the grouping's capacity, it reads the padded row count
+// from device memory and the threads past it exit
+__global__ void __launch_bounds__(256) k_gather_obs_rows_dev(const uint4* __restrict__ src, const int32_t* __restrict__ index,
+                                                             uint4* __restrict__ dst, const int32_t* __restrict__ n_rows, int w) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)*n_rows * w) return;
+    const int64_t r = i / w;
+    const int c = (int)(i - r * w);
+    const int32_t e = index[r];
+    dst[i] = e >= 0 ? src[(int64_t)e * w + c] : make_uint4(0u, 0u, 0u, 0u);
 }
 
 }  // namespace brl
@@ -906,7 +969,7 @@ static bool fused_forward(const BrlParams* p) {
 // forward (+ optional fused categorical) shared by brl_mlp_forward and brl_policy_act.  GROUPED (brl_policy_act_grouped): `blob`
 // is a pool of nets, row block b of the batch runs net pool->block_model[b], and the head epilogue writes action / logits by env
 // (the per-layer head included: no categorical launch).
-template <bool GROUPED = false>
+template <bool GROUPED = false, bool DEVCOUNT = false>
 static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams* p, const void* obs, const unsigned char* blob,
                                 __nv_bfloat16* scratch, float* logits, float* value, const ActArgs& act, const PoolArgs* pool = nullptr) {
     int32_t rc = BRL_OK;
@@ -920,8 +983,8 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
     __nv_bfloat16* buf_lo[2] = {scratch + 2 * act_elems, scratch + 3 * act_elems};
     if (fused_forward(p)) {
         uint32_t* ready = reinterpret_cast<uint32_t*>(scratch + 4 * act_elems);
-        rc = split ? launch_fused<true, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
-                   : launch_fused<false, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
+        rc = split ? launch_fused<true, GROUPED, DEVCOUNT>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
+                   : launch_fused<false, GROUPED, DEVCOUNT>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
         if (rc != BRL_OK) return rc;
         return check_launch(who);
     }
@@ -943,16 +1006,16 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
             a.out_lo = split ? buf_lo[l & 1] : nullptr;
             // 128 x 256 tiles move fewer operand bytes per MMA (the L2 -> SM fill rate, ~64 B/clk, is what bounds
             // these 1-CTA tiles): measured faster for the single-product mode; the split mode runs 128 x 128 tiles
-            if (!split) rc = launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            else if (l == 0) rc = launch_layer<128, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            else rc = launch_layer<128, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            if (!split) rc = launch_layer<256, false, false, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else if (l == 0) rc = launch_layer<128, false, true, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else rc = launch_layer<128, true, true, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
             in_hi = a.out_hi;
             in_lo = a.out_lo;
         } else {
             a.logits = GROUPED ? logits : lg;
             a.value = GROUPED ? nullptr : vl;
-            rc = split ? launch_layer<kHeadPad, true, true, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool)
-                       : launch_layer<kHeadPad, false, false, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool);
+            rc = split ? launch_layer<kHeadPad, true, true, true, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool)
+                       : launch_layer<kHeadPad, false, false, true, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool);
         }
         if (rc != BRL_OK) return rc;
     }
@@ -1105,3 +1168,47 @@ int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t
 }
 
 }  // extern "C"
+
+namespace brl {
+
+// ---- the grouped forward of brl_duplicate_match's device loop (brl_match.cu) ------------------------------------------------
+// brl_policy_act_grouped with the padded row count in device memory (`n_rows` = brl_model_rows' offsets[M]): the gather, the
+// launches and their tensor maps are sized for `capacity` rows, and the DEVCOUNT kernels stop at the count.  The caller picks the
+// path: `flags` holds BRL_F_TUNE_MLP_LAYERS or BRL_F_TUNE_MLP_FUSED (and BRL_F_MLP_BF16 for the single-product mode).
+int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
+                                  const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
+                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows) {
+    BrlParams p{};
+    p.n_envs = capacity;
+    p.flags = flags;
+    p.k_steps = n_models;
+    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(capacity));
+    const int w = kObsDimM * 2 / 16;
+    k_gather_obs_rows_dev<<<(unsigned)((capacity * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(obs), rows, gathered,
+                                                                                 n_rows, w);
+    ActArgs act{};
+    act.mask = mask;
+    act.action = action;
+    act.row_index = rows;
+    const PoolArgs pa{block_model, brl_mlp_pool_stride(), n_models, act, n_rows};
+    return mlp_forward_impl<true, true>("brl_duplicate_match", s, &p, gathered, pool, reinterpret_cast<__nv_bfloat16*>(scratch),
+                                        nullptr, nullptr, act, &pa);
+}
+
+// everything launch_policy_grouped_dev sets up once per device -- the driver's tensor-map entry point, the kernels'
+// shared-memory attributes, the fused kernel's co-resident pair count -- done before a stream capture begins
+int32_t warm_policy_grouped_dev(bool split) {
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_duplicate_match: cuTensorMapEncodeTiled not available from the driver");
+    int32_t rc;
+    if (split) {
+        if ((rc = layer_attr<128, false, true, false, true, true>()) || (rc = layer_attr<128, true, true, false, true, true>()) ||
+            (rc = layer_attr<kHeadPad, true, true, true, true, true>()))
+            return rc;
+        return fused_pairs<true, true, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
+    }
+    if ((rc = layer_attr<256, false, false, false, true, true>()) || (rc = layer_attr<kHeadPad, false, false, true, true, true>()))
+        return rc;
+    return fused_pairs<false, true, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
+}
+
+}  // namespace brl

@@ -63,6 +63,10 @@ inline int sm_count() {
 // the row tile of the fused forward's CTA pairs, so that no tile mixes two nets.
 constexpr int kGroupRows = 256;
 
+// batches from this size on run the policy forward as one fused launch on CTA pairs (brl_mlp.cu fused_forward; also the rule
+// brl_duplicate_match's device loop applies to its device-side row count)
+constexpr int kPairMinM = 4096;
+
 // masked categorical over f32 logits[n,38] (brl_algo.cu); shared by brl_categorical and the unfused brl_policy_act path
 int32_t launch_categorical(cudaStream_t stream, const float* logits, const unsigned char* mask, int32_t* action, float* log_prob,
                            int64_t n, int sample, uint64_t seed, int64_t env_offset, uint32_t step, const int32_t* row_index = nullptr,

@@ -13,7 +13,6 @@ constexpr int kObsDimM = 480, kHidden = 1024, kHeadValid = 39, kHeadPad = 64;
 constexpr int kBM = 128, kBK = 64, kUmmaK = 16;
 constexpr int kMlpThreads = 192;
 constexpr uint32_t kSmemBudget = 200 * 1024;
-constexpr int kPairMinM = 4096;  // batches from this size on run the hidden layers on CTA pairs
 
 // ---- packed parameter blob ---------------------------------------------------------------
 struct MlpLayout {

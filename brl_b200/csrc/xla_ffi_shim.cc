@@ -74,6 +74,7 @@
     X(brl_model_rows, "iiioooo") \
     X(brl_policy_act_grouped, "iisixiix") \
     X(brl_match_stats_ranges, "iix") \
+    X(brl_duplicate_match, "iiiiisoxooooooooooooo") \
     /* end */
 
 namespace {

@@ -280,6 +280,123 @@ def _league_chunk(eval_env, keys, env_models, pool, single_bf16, counter):
     return cum_return
 
 
+# ---- the device-loop evaluators: one brl_duplicate_match call per match / league chunk (eval.py:53) -------------------------
+class _MatchBuffers:
+    """Fixed-address inputs and outputs of brl_duplicate_match for one shape (n envs, M nets, P ranges; P = 0: one range
+    over the batch), so that repeated calls relaunch the op's cached graph instead of capturing a new one."""
+
+    def __init__(self, n: int, M: int, P: int, dev, with_models: bool, with_tables: bool):
+        self.keys = torch.empty(n, dtype=torch.int64, device=dev)
+        self.pool = torch.zeros((M, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
+        self.env_models = torch.empty((n, 2), dtype=torch.int32, device=dev) if with_models else None
+        self.offsets = torch.empty(P + 1, dtype=torch.int64, device=dev) if P else None
+        self.scratch = torch.empty(ops.duplicate_match_scratch_bytes(n, M), dtype=torch.uint8, device=dev)
+        self.cum_return = torch.empty(n, dtype=torch.float32, device=dev)
+        self.sums = torch.zeros((P, 8) if P else (8,), dtype=torch.float64, device=dev)
+        self.status = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.tables = (ops.TableInfoBuffers(n, dev), ops.TableInfoBuffers(n, dev)) if with_tables else (None, None)
+
+    def play(self, eval_env, single_bf16: bool, tune: int):
+        self.sums.zero_()
+        ops.duplicate_match(self.keys, eval_env.table, self.pool, self.scratch, self.cum_return, self.sums, self.status,
+                            env_models=self.env_models, range_offsets=self.offsets, table_a=self.tables[0],
+                            table_b=self.tables[1], single_bf16=single_bf16, tune=tune,
+                            illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
+
+
+def _check_match_status(status: int) -> None:
+    if status == ops._lib.MATCH_BAD_MODEL:
+        raise ops._lib.BrlError("brl_duplicate_match: an acting net id is outside [0, M)")
+    if status != ops._lib.MATCH_OK:
+        raise ops._lib.BrlError(f"brl_duplicate_match: envs still live after {ops._lib.MATCH_MAX_STEPS} steps (status {status})")
+
+
+def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_envs, env_offset: int = 0, *, tune: int = 0):
+    """make_simple_duplicate_evaluate (src/evaluation.py:69-204) with the whole match in one brl_duplicate_match call: the
+    loop runs on the device (a CUDA graph WHILE node), so a match costs one launch and one host read of its statistics.
+    Same contract -- `duplicate_evaluate(team1_params, team2_params, rng_key) -> (log_info, table_a_info, table_b_info,
+    cum_return)`, same key split and keys, one all-reduce of f64[8] over the ranks -- and the same per-env results.
+    Both teams share `activation` / `model_type` (the pool holds one architecture).  `record` / `trace` need per-step host
+    copies: use make_simple_duplicate_evaluate for them.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path."""
+    forward_pass = make_forward_pass(activation=activation, model_type=model_type)
+    n, dev = num_eval_envs, eval_env.device
+    bufs = _MatchBuffers(n, 2, 0, dev, with_models=False, with_tables=True)
+    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+
+    def duplicate_evaluate(team1_params, team2_params, rng_key):
+        rng_key, sub_key = brandom.split(rng_key)
+        bufs.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))                       # :93-94
+        forward_pass.pack_into(team1_params, bufs.pool[0, :blob_bytes])
+        forward_pass.pack_into(team2_params, bufs.pool[1, :blob_bytes])
+        bufs.play(eval_env, forward_pass.precision == "tc-bf16", tune)                      # :95-198
+        sums = bufs.sums.clone()
+        bdist.allreduce_sums(sums)
+        host = torch.cat((sums, bufs.status.to(torch.float64))).cpu()
+        _check_match_status(int(host[8]))
+        log_info = bdist.stats_from_sums(host[:8])                                        # :199-201
+        infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
+                            t.call_xx.clone()) for t in bufs.tables]
+        return log_info, infos[0], infos[1], bufs.cum_return.clone()
+
+    return duplicate_evaluate
+
+
+def make_device_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *,
+                                         tune: int = 0):
+    """make_selfplay_league_evaluate with one brl_duplicate_match call per chunk: the same pairs, chunks, sharding and
+    all-reduce, the same per-env returns, statistics and matrices, with each chunk's loop on the device."""
+    import itertools
+
+    import numpy as np
+    forward_pass = make_forward_pass(activation=activation, model_type=model_type)
+    rank, world = bdist.rank_world()
+    n, dev = num_eval_envs, eval_env.device
+    pairs_per_chunk = max(1, (max_envs * world) // n)
+    buffers = {}
+    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+
+    def league(params_list, rng_key, cum_returns=None):
+        M = len(params_list)
+        pairs = list(itertools.combinations(range(M), 2))
+        _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
+        board_keys = eval_env.make_keys(sub_key, n)
+        stats = {}
+        for c0 in range(0, len(pairs), pairs_per_chunk):
+            chunk = pairs[c0:c0 + pairs_per_chunk]
+            P = len(chunk)
+            lo, hi = bdist.shard_range(P * n, rank, world)
+            sums = torch.zeros((P, 8), dtype=torch.float64, device=dev)
+            status = 0
+            if hi > lo:
+                g = np.arange(lo, hi)
+                pair_arr = np.asarray(chunk, dtype=np.int32)
+                p_lo, p_hi = lo // n, (hi + n - 1) // n                                  # the matches this shard touches
+                bounds = np.clip(np.arange(p_lo, p_hi + 1, dtype=np.int64) * n - lo, 0, hi - lo)  # their local env ranges
+                key = (hi - lo, M, p_hi - p_lo)
+                if key not in buffers:
+                    buffers[key] = _MatchBuffers(hi - lo, M, p_hi - p_lo, dev, with_models=True, with_tables=False)
+                b = buffers[key]
+                for m, params in enumerate(params_list):
+                    forward_pass.pack_into(params, b.pool[m, :blob_bytes])
+                b.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
+                b.env_models.copy_(torch.as_tensor(pair_arr[g // n], device=dev))
+                b.offsets.copy_(torch.as_tensor(bounds, device=dev))
+                b.play(eval_env, forward_pass.precision == "tc-bf16", tune)
+                sums[p_lo:p_hi] = b.sums
+                status = b.status
+                if cum_returns is not None:
+                    for p in range(p_lo, p_hi):
+                        cum_returns[chunk[p]] = b.cum_return[int(bounds[p - p_lo]):int(bounds[p - p_lo + 1])].clone()
+            bdist.allreduce_sums(sums)
+            host = sums.cpu()
+            _check_match_status(int(status))
+            for p, pair in enumerate(chunk):
+                stats[pair] = bdist.stats_from_sums(host[p])
+        return (stats,) + league_matrices(M, {pair: s[0] for pair, s in stats.items()})
+
+    return league
+
+
 # ---- full evaluation statistics (src/evaluation.py:207-1115) --------------------------------------
 _S_TABLE, _S_BIDS, _S_CONTRACTS = 11, 29, 99
 

@@ -559,3 +559,53 @@ def match_stats_ranges(x: torch.Tensor, offsets: torch.Tensor, sums: torch.Tenso
     if offsets.dtype != torch.int64 or sums.dtype != torch.float64 or tuple(sums.shape) != (offsets.shape[0] - 1, 8):
         raise _lib.BrlError("match_stats_ranges: offsets must be int64[P + 1] and sums float64[P, 8]")
     _call("brl_match_stats_ranges", [_ptr(x), _ptr(offsets), _ptr(sums)], _params(sums.shape[0]))
+
+
+# ---- a whole duplicate match as one call (eval.py:53, src/evaluation.py:69-204) -------------------------------------------
+def duplicate_match_scratch_bytes(n_envs: int, n_models: int) -> int:
+    return _size_query("brl_duplicate_match_scratch_bytes", n_envs, n_models)
+
+
+def duplicate_match_graph_builds() -> int:
+    """graphs brl_duplicate_match has captured and instantiated in this process (a repeated call with the same buffers and
+    parameters relaunches its cached graph)"""
+    fn = _lib.load().brl_duplicate_match_graph_builds
+    fn.restype, fn.argtypes = _lib.C.c_longlong, []
+    return int(fn())
+
+
+def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, cum_return: torch.Tensor,
+                    sums: torch.Tensor, status: torch.Tensor, *, env_models: Optional[torch.Tensor] = None,
+                    range_offsets: Optional[torch.Tensor] = None, table_a: Optional[TableInfoBuffers] = None,
+                    table_b: Optional[TableInfoBuffers] = None, single_bf16: bool = False, tune: int = 0,
+                    illegal_penalty: float = -1.0, illegal_bonus: float = 1.0) -> None:
+    """Play duplicate_evaluate's whole loop (src/evaluation.py:93-201) for every env of `keys` in one call, with the loop on
+    the device: env e plays net env_models[e, 0] of `pool` on players 0/1 against env_models[e, 1] on 2/3 (default: net 0
+    against net 1, M must be 2).  Writes cum_return f32[n], adds the match sums to `sums` (f64[P, 8] over the ranges of
+    `range_offsets` int64[P + 1], or f64[8] for the whole batch), the status (int32[1], _lib.MATCH_*) and, when given, the
+    final Table_info of both tables.  Nothing is read back to the host; read `status` with the sums."""
+    n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
+    if env_models is None and M != 2:
+        raise _lib.BrlError(f"duplicate_match: without env_models the pool must hold 2 nets, got {M}")
+    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) != (n, 2)):
+        raise _lib.BrlError("duplicate_match: env_models must be int32 [n, 2]")
+    P = 0
+    if range_offsets is not None:
+        P = int(range_offsets.shape[0]) - 1
+        if range_offsets.dtype != torch.int64 or P < 1 or tuple(sums.shape) != (P, 8):
+            raise _lib.BrlError("duplicate_match: range_offsets must be int64[P + 1] with sums float64[P, 8]")
+    elif sums.numel() != 8:
+        raise _lib.BrlError("duplicate_match: without range_offsets sums is float64[8]")
+    if sums.dtype != torch.float64 or cum_return.dtype != torch.float32 or status.dtype != torch.int32:
+        raise _lib.BrlError("duplicate_match: sums must be float64, cum_return float32 and status int32")
+    if pool.dim() != 2 or pool.dtype != torch.uint8 or pool.shape[1] != mlp_pool_stride():
+        raise _lib.BrlError("duplicate_match: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    if scratch.numel() < duplicate_match_scratch_bytes(n, M):
+        raise _lib.BrlError("duplicate_match: scratch too small (ops.duplicate_match_scratch_bytes)")
+    if (table_a is None) != (table_b is None):
+        raise _lib.BrlError("duplicate_match: give both Table_info outputs or neither")
+    infos = table_a.ptrs() + table_b.ptrs() if table_a is not None else [None] * 12
+    _call("brl_duplicate_match", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(env_models), _ptr(range_offsets), _ptr(scratch),
+                                  _ptr(cum_return), _ptr(sums), _ptr(status)] + infos,
+          _params(n, k_steps=M, step=P, n_deals=table.shape[0], flags=(F_MLP_BF16 if single_bf16 else 0) | tune,
+                  illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))

@@ -64,6 +64,8 @@
  *   brl_policy_act_grouped  team{1,2}_forward_pass.apply + masked argmax of every match of a league, one forward over a
  *                         pool of nets                 workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
  *   brl_match_stats_ranges  brl_match_stats of every match of a league chunk   src/evaluation.py:199-201
+ *   brl_duplicate_match   jax.jit(make_simple_duplicate_evaluate(...)) as one call: init, Table_info, the whole
+ *                         lax.while_loop and the match sums   eval.py:53 ; src/evaluation.py:69-204
  */
 #ifndef BRL_B200_H
 #define BRL_B200_H
@@ -296,6 +298,37 @@ int32_t brl_policy_act_grouped(brl_stream_t, void **buffers, const void *opaque,
  *          [2] inout f64 sums[P, 8] */
 int32_t brl_match_stats_ranges(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- a whole duplicate match as one call (eval.py:53, src/evaluation.py:69-204) ---------------------------------------
+ * make_simple_duplicate_evaluate's duplicate_evaluate for every env of the batch, with the loop on the device:
+ *   brl_init from the keys (:93-95) -> Table_info A = B from the init state (:97-112) -> while any env is live { live rows
+ *   grouped by acting net (brl_model_rows, :124-151) -> masked-argmax forward of every net of the pool
+ *   (brl_policy_act_grouped, :124-133) -> brl_duplicate_step (:164) -> cum_return += rewards[:, 0] (:167-169) } ->
+ *   sums += brl_match_stats per env range (:199-201).
+ * The loop is a CUDA graph WHILE node whose condition a kernel sets from the padded row count on the device; the forward
+ * takes its row count from device memory too, and its path follows brl_policy_act's rule on that count (one fused launch
+ * from 4096 rows on, per-layer launches below; BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED pin one).  Nothing is read
+ * back to the host.  On a plain stream the call captures the match once per set of buffers and params into a graph it
+ * keeps (repeated calls with the same buffers relaunch it; brl_duplicate_match_graph_builds() counts the builds); on a
+ * stream that is being captured (a CUDA graph, an XLA command buffer) it adds the same nodes to the caller's capture.
+ * Unlike the other ops it keeps this cache and three private capture streams per device, created on the first call;
+ * make that first call outside a capture.
+ * buffers: [0] in u64 keys[n] (brl_make_keys)  [1] in deal_table  [2] in pool u8[M, brl_mlp_pool_stride()]
+ *          [3] in i32 env_models[n,2] (NULL: M must be 2, every env plays net 0 on players 0/1 against net 1 on 2/3)
+ *          [4] in i64 range offsets[P + 1] (NULL: one range, the whole batch)  [5] scratch
+ *          (brl_duplicate_match_scratch_bytes(n, M))  [6] out f32 cum_return[n]  [7] inout f64 sums[P, 8] (+=, as
+ *          brl_match_stats_ranges; sums[8] for one range)  [8] out i32 status[1] (BRL_MATCH_*)
+ *          [9..14] out final Table_info A {u8 terminated, f32 rewards[n,4], i32 last_bid, i32 last_bidder, u8 call_x,
+ *          u8 call_xx}  [15..20] out Table_info B -- all twelve or none (then they live in the scratch)
+ * params: n_envs = n, k_steps = M, step = P (0 with [4] NULL), n_deals, illegal_penalty / illegal_bonus as brl_step,
+ *         flags BRL_F_MLP_BF16 / BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED (BRL_F_SAMPLE is an error). */
+#define BRL_MATCH_MAX_STEPS 638    /* an auction has at most 319 calls; an env finishes both tables in at most 638 steps */
+#define BRL_MATCH_OK 0
+#define BRL_MATCH_BAD_MODEL 1      /* a live env's acting net id is outside [0, M): the loop stopped, outputs invalid */
+#define BRL_MATCH_STEP_BOUND 2     /* envs still live after BRL_MATCH_MAX_STEPS forwards: the loop stopped */
+int64_t brl_duplicate_match_scratch_bytes(int64_t n_envs, int64_t n_models);
+long long brl_duplicate_match_graph_builds(void);
+int32_t brl_duplicate_match(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -485,6 +518,7 @@ void brl_team_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t 
 void brl_model_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_policy_act_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_match_stats_ranges_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_duplicate_match_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_loss_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_clip_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_apply_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
