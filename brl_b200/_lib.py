@@ -15,7 +15,7 @@ from . import build as _build
 # eagerly moved the interpreter's garbage-collection schedule in bench.py so that its rollout leg measured 8 % slower on a
 # B200 (1000 W), with identical device code and identical timings under gc.disable().
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
-            "brl_duplicate_match")
+            "brl_duplicate_match", "brl_evaluate_match")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -30,7 +30,7 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_xla_layout", "brl_xla_unreported_failures", "brl_eval_num_sums",
         "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset",
         "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes",
-        "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds")
+        "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 
@@ -55,6 +55,13 @@ EVAL_ACC_COLS = 76
 MATCH_MAX_STEPS = 638  # brl_duplicate_match's bound on forwards (BRL_MATCH_MAX_STEPS)
 MATCH_OK, MATCH_BAD_MODEL, MATCH_STEP_BOUND = 0, 1, 2  # its status codes (BRL_MATCH_*)
 F_TUNE_MLP_LAYERS, F_TUNE_MLP_FUSED = 1 << 29, 1 << 30  # pin the policy forward's path (BRL_F_TUNE_MLP_*)
+EVAL_MATCH_DUPLICATE, EVAL_MATCH_SINGLE, EVAL_MATCH_SIMPLE = 1, 2, 3  # brl_evaluate_match's modes (BRL_EVAL_MATCH_*)
+F_EVAL_FREE_RUN = 0x0008  # brl_evaluate_match: team 2 always passes (BRL_F_EVAL_FREE_RUN)
+
+
+def f_eval_match(mode: int) -> int:
+    """BRL_F_EVAL_MATCH(mode): the flag bits naming brl_evaluate_match's mode"""
+    return mode << 27
 
 
 def tune(epw: int = 0, wpb: int = 0, classic_rollout: bool = False, writers: int = 0, balanced=None) -> int:

@@ -1,6 +1,9 @@
-// brl_match.cu -- a whole duplicate match as one stream-ordered call (brl_duplicate_match): make_simple_duplicate_evaluate
-// (src/evaluation.py:69-204) for every env of the batch, its `lax.while_loop` (:120-171) run on the device by a CUDA graph
-// WHILE node.  sm_100a only.
+// brl_match.cu -- a whole evaluation as one stream-ordered call, its `lax.while_loop` run on the device by a CUDA graph WHILE
+// node.  sm_100a only.
+//   brl_duplicate_match   make_simple_duplicate_evaluate (src/evaluation.py:69-204) for every env of the batch
+//   brl_evaluate_match    make_evaluate's duplicate / single-table evaluate (:207-1032) and make_simple_evaluate (:11-66):
+//                         the same loop with the step log (brl_eval_act_log) and the statistics (brl_eval_summary), or with
+//                         one env step per iteration and the actor's return
 //
 //   init (brl_init) -> Table_info A / B (brl_state_fields) -> grouping (brl_model_rows) -> control
 //   WHILE (control said so) {
@@ -8,6 +11,9 @@
 //       brl_duplicate_step -> cum_return += rewards[:, 0] -> grouping -> control
 //   }
 //   match sums (brl_match_stats_ranges, or brl_match_stats for one range)
+//
+// brl_evaluate_match runs the same skeleton: its body adds brl_eval_act_log after the forward (full statistics), steps with
+// brl_step instead of brl_duplicate_step where there is one table, and ends with brl_eval_summary (or nothing: simple).
 //
 // The control kernel reads the padded row count brl_model_rows left in offsets[M] and sets the loop's condition: the loop
 // ends when no env is live, when a live env's net id is outside [0, M), or at BRL_MATCH_MAX_STEPS forwards; the last two
@@ -29,7 +35,7 @@ namespace brl {
 
 int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
                                   const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
-                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows);
+                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits);
 int32_t warm_policy_grouped_dev(bool split);
 
 // ---- kernels -----------------------------------------------------------------------------------------------------------
@@ -41,6 +47,37 @@ __global__ void __launch_bounds__(256) k_pair_models(int32_t* __restrict__ env_m
 __global__ void __launch_bounds__(256) k_add_reward(float* __restrict__ cum_return, const float4* __restrict__ rewards, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) cum_return[i] += rewards[i].x;  // cum_return += state.rewards[:, 0] (src/evaluation.py:167-169)
+}
+
+// make_simple_evaluate: the actor (net 0) decides for the team of the env's initial player, the opponent (net 1) for the other
+// (src/utils.py:133-202: actor, opp, actor, opp from the player to act at the quad step's start), and R gathers that player's reward
+__global__ void __launch_bounds__(256) k_actor_models(int32_t* __restrict__ env_models, int8_t* __restrict__ actor,
+                                                      const int8_t* __restrict__ player, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int8_t p = player[i];
+    actor[i] = p;
+    reinterpret_cast<int2*>(env_models)[i] = p < 2 ? make_int2(0, 1) : make_int2(1, 0);
+}
+
+__global__ void __launch_bounds__(256) k_add_actor_reward(float* __restrict__ R, const float* __restrict__ rewards,
+                                                          const int8_t* __restrict__ actor, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) R[i] += rewards[4 * i + actor[i]];  // R + rewards[actor] (src/evaluation.py:60); non-zero on the last step only
+}
+
+__global__ void __launch_bounds__(256) k_sum_rewards(float* __restrict__ cum_return, float4* __restrict__ rewards_sum,
+                                                     const float4* __restrict__ rewards, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 r = rewards[i];
+    float4 s = rewards_sum[i];
+    s.x += r.x;
+    s.y += r.y;
+    s.z += r.z;
+    s.w += r.w;
+    rewards_sum[i] = s;  // rewards += state.rewards, cum_return += rewards[:, 0] (src/evaluation.py:407-411)
+    cum_return[i] += r.x;
 }
 
 // after each grouping: continue while rows are live; stop with a status on a bad net id or at the step bound.  `iter` counts
@@ -67,12 +104,13 @@ __global__ void k_match_path(const int32_t* __restrict__ n_rows, cudaGraphCondit
 }
 
 // ---- the scratch ----------------------------------------------------------------------------------------------------------
+// brl_duplicate_match's pieces; brl_evaluate_match (mode > 0) appends its own behind them
 struct MatchLayout {
     size_t state, obs, mask, rewards, terminated, player, action, info[2][6], env_models, rows, counts, offsets, block_model, ctl,
-        forward, total;
+        forward, logits, fields[6], rewards_sum, actor, total;
 };
 
-static MatchLayout match_layout(int64_t n, int64_t M) {
+static MatchLayout match_layout(int64_t n, int64_t M, int mode = 0) {
     MatchLayout L{};
     size_t off = 0;
     auto take = [&](size_t bytes) {
@@ -103,12 +141,22 @@ static MatchLayout match_layout(int64_t n, int64_t M) {
     L.block_model = take(cap / kGroupRows * 4);
     L.ctl = take(16);  // i32 iteration counter
     L.forward = take((size_t)brl_policy_grouped_scratch_bytes(n, M));
+    if (mode == BRL_EVAL_MATCH_DUPLICATE || mode == BRL_EVAL_MATCH_SINGLE) {
+        L.logits = take(un * BRL_NUM_ACTIONS * 4);
+        for (int k = 0; k < 4; ++k) L.fields[k] = take(un * 4);  // i32 step_count, last_bid, last_bidder, pass_num
+        for (int k = 4; k < 6; ++k) L.fields[k] = take(un);      // u8 call_x, call_xx
+    }
+    if (mode == BRL_EVAL_MATCH_SINGLE) L.rewards_sum = take(un * 16);
+    if (mode == BRL_EVAL_MATCH_SIMPLE) L.actor = take(un);
     L.total = off;
     return L;
 }
 
 // every device pointer and size one match needs
 struct MatchPlan {
+    const char* who;  // the op, for error messages
+    int mode;         // 0: brl_duplicate_match; else BRL_EVAL_MATCH_*
+    bool free_run;    // brl_evaluate_match: team 2 always passes
     int64_t n, cap, P;
     int M;
     int32_t n_deals, flags;
@@ -124,6 +172,10 @@ struct MatchPlan {
     MatchLayout L;
     int32_t* env_models;  // the caller's, or (NULL given) the scratch's, filled with net 0 vs net 1
     bool default_models;
+    void *state, *obs, *mask, *terminated, *player;  // the loop's env buffers: the scratch's, or the caller's final-state outputs
+    float* logits;       // full statistics: the acting net's logits by env, for brl_eval_act_log (else NULL)
+    float* acc;          // full statistics: the per-env log rows
+    float* rewards_sum;  // single table: sum of the step rewards
     template <class T = void>
     T* at(size_t off) const { return reinterpret_cast<T*>(scratch + off); }
     int32_t* offsets() const { return at<int32_t>(L.offsets); }
@@ -140,15 +192,22 @@ static BrlParams env_params(const MatchPlan& q, int64_t n) {
     return p;
 }
 
-// a failed graph-building call: its CUDA error, or a plain failure when the call left none
-static int32_t launch_error(const char* what) {
-    const int32_t rc = check_launch(what);
-    return rc != BRL_OK ? rc : fail(BRL_E_LAUNCH, "%s failed", what);
+// check_launch for one step of `who`
+static int32_t launched(const char* who, const char* step) {
+    const cudaError_t err = cudaGetLastError();
+    return err == cudaSuccess ? BRL_OK : fail(BRL_E_LAUNCH, "%s (%s): %s", who, step, cudaGetErrorString(err));
 }
 
+// a failed graph-building call: its CUDA error, or a plain failure when the call left none
+static int32_t launch_error(const char* who, const char* step) {
+    const int32_t rc = launched(who, step);
+    return rc != BRL_OK ? rc : fail(BRL_E_LAUNCH, "%s (%s) failed", who, step);
+}
+
+static unsigned blocks(int64_t n) { return (unsigned)((n + 255) / 256); }
+
 static int32_t model_rows(const MatchPlan& q, cudaStream_t s) {
-    void* b[7] = {q.at(q.L.player), q.at(q.L.terminated), q.env_models, q.at(q.L.rows), q.at(q.L.counts), q.offsets(),
-                  q.at(q.L.block_model)};
+    void* b[7] = {q.player, q.terminated, q.env_models, q.at(q.L.rows), q.at(q.L.counts), q.offsets(), q.at(q.L.block_model)};
     BrlParams p = env_params(q, q.n);
     p.k_steps = q.M;
     return brl_model_rows(s, b, &p, sizeof(p));
@@ -156,18 +215,19 @@ static int32_t model_rows(const MatchPlan& q, cudaStream_t s) {
 
 static int32_t control(const MatchPlan& q, cudaStream_t s, cudaGraphConditionalHandle loop) {
     k_match_control<<<1, 1, 0, s>>>(q.offsets() + q.M, q.at<int32_t>(q.L.ctl), q.status, loop);
-    return check_launch("brl_duplicate_match (control)");
+    return launched(q.who, "control");
 }
 
 // the capture's graph, with the stream's current dependencies; a conditional node of `type` there (its body in *body), made
 // the stream's only dependency
-static int32_t add_conditional(cudaStream_t s, cudaGraphConditionalHandle h, cudaGraphConditionalNodeType type, cudaGraph_t* body) {
+static int32_t add_conditional(const char* who, cudaStream_t s, cudaGraphConditionalHandle h, cudaGraphConditionalNodeType type,
+                               cudaGraph_t* body) {
     cudaStreamCaptureStatus st;
     cudaGraph_t g = nullptr;
     const cudaGraphNode_t* deps = nullptr;
     size_t n_deps = 0;
     if (cudaStreamGetCaptureInfo(s, &st, nullptr, &g, &deps, &n_deps) != cudaSuccess || st != cudaStreamCaptureStatusActive)
-        return launch_error("brl_duplicate_match (capture info)");
+        return launch_error(who, "capture info");
     cudaGraphNodeParams cp{};
     cp.type = cudaGraphNodeTypeConditional;
     cp.conditional.handle = h;
@@ -176,41 +236,64 @@ static int32_t add_conditional(cudaStream_t s, cudaGraphConditionalHandle h, cud
     cudaGraphNode_t node;
     if (cudaGraphAddNode(&node, g, deps, n_deps, &cp) != cudaSuccess ||
         cudaStreamUpdateCaptureDependencies(s, &node, 1, cudaStreamSetCaptureDependencies) != cudaSuccess)
-        return launch_error("brl_duplicate_match (conditional node)");
+        return launch_error(who, "conditional node");
     *body = cp.conditional.phGraph_out[0];
     return BRL_OK;
 }
 
-static int32_t new_handle(cudaStream_t s, cudaGraphConditionalHandle* h) {
+static int32_t new_handle(const char* who, cudaStream_t s, cudaGraphConditionalHandle* h) {
     cudaStreamCaptureStatus st;
     cudaGraph_t g = nullptr;
     if (cudaStreamGetCaptureInfo(s, &st, nullptr, &g) != cudaSuccess || st != cudaStreamCaptureStatusActive ||
         cudaGraphConditionalHandleCreate(h, g, 0, cudaGraphCondAssignDefault) != cudaSuccess)
-        return launch_error("brl_duplicate_match (conditional handle)");
+        return launch_error(who, "conditional handle");
     return BRL_OK;
 }
 
 // fill `body` by capturing what `fn(side)` enqueues on the side stream
 template <class F>
-static int32_t capture_into(cudaGraph_t body, cudaStream_t side, F&& fn) {
+static int32_t capture_into(const char* who, cudaGraph_t body, cudaStream_t side, F&& fn) {
     if (cudaStreamBeginCaptureToGraph(side, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed) != cudaSuccess)
-        return launch_error("brl_duplicate_match (body capture)");
+        return launch_error(who, "body capture");
     const int32_t rc = fn(side);
     cudaGraph_t out = nullptr;
     const cudaError_t end = cudaStreamEndCapture(side, &out);
     if (rc != BRL_OK) return rc;
-    if (end != cudaSuccess) return launch_error("brl_duplicate_match (body capture)");
+    if (end != cudaSuccess) return launch_error(who, "body capture");
     return BRL_OK;
 }
 
 static int32_t forward(const MatchPlan& q, cudaStream_t s, int32_t path_flag) {
     const int32_t flags = (q.flags & BRL_F_MLP_BF16) | path_flag;
-    return launch_policy_grouped_dev(s, flags, q.cap, q.M, q.at(q.L.obs), q.pool, q.at<unsigned char>(q.L.forward),
-                                     q.at<uint8_t>(q.L.mask), q.at<int32_t>(q.L.action), q.at<int32_t>(q.L.rows),
-                                     q.at<int32_t>(q.L.block_model), q.offsets() + q.M);
+    return launch_policy_grouped_dev(s, flags, q.cap, q.M, q.obs, q.pool, q.at<unsigned char>(q.L.forward), static_cast<uint8_t*>(q.mask),
+                                     q.at<int32_t>(q.L.action), q.at<int32_t>(q.L.rows), q.at<int32_t>(q.L.block_model),
+                                     q.offsets() + q.M, q.logits);
 }
 
-// one iteration of the loop (src/evaluation.py:124-169), on the body's capture stream s1; s2 captures the IF bodies
+// the env step of one iteration: brl_duplicate_step on both tables (:164, :772-774), or brl_step without auto-reset (:406;
+// make_simple_evaluate: src/utils.py:133-202 one sub-step at a time)
+static int32_t env_step(const MatchPlan& q, cudaStream_t s) {
+    const BrlParams p = env_params(q, q.n);
+    void* const action = q.at(q.L.action);
+    if (q.mode == BRL_EVAL_MATCH_SINGLE || q.mode == BRL_EVAL_MATCH_SIMPLE) {
+        void* b[10] = {q.state, action, const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated, q.player,
+                       nullptr};
+        return brl_step(s, b, &p, sizeof(p));
+    }
+    void* b[21] = {q.state, action, const_cast<void*>(q.table)};
+    for (int t = 0; t < 2; ++t)
+        for (int k = 0; k < 6; ++k) b[3 + 6 * t + k] = q.info[t][k];
+    b[15] = q.state;
+    b[16] = q.obs;
+    b[17] = q.mask;
+    b[18] = q.at(q.L.rewards);
+    b[19] = q.terminated;
+    b[20] = q.player;
+    return brl_duplicate_step(s, b, &p, sizeof(p));
+}
+
+// one iteration of the loop (src/evaluation.py:124-169; :388-411 / :748-777 with the step log; :42-61), on the body's capture
+// stream s1; s2 captures the IF bodies
 static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, cudaGraphConditionalHandle loop) {
     int32_t rc;
     if (q.flags & BRL_F_TUNE_MLP_LAYERS) {
@@ -219,66 +302,112 @@ static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, c
         rc = forward(q, s1, BRL_F_TUNE_MLP_FUSED);
     } else {
         cudaGraphConditionalHandle h_fused, h_layers;
-        if ((rc = new_handle(s1, &h_fused)) || (rc = new_handle(s1, &h_layers))) return rc;
+        if ((rc = new_handle(q.who, s1, &h_fused)) || (rc = new_handle(q.who, s1, &h_layers))) return rc;
         k_match_path<<<1, 1, 0, s1>>>(q.offsets() + q.M, h_fused, h_layers);
-        if ((rc = check_launch("brl_duplicate_match (path)"))) return rc;
+        if ((rc = launched(q.who, "path"))) return rc;
         cudaGraph_t body;
-        if ((rc = add_conditional(s1, h_fused, cudaGraphCondTypeIf, &body)) ||
-            (rc = capture_into(body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_FUSED); })) ||
-            (rc = add_conditional(s1, h_layers, cudaGraphCondTypeIf, &body)) ||
-            (rc = capture_into(body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_LAYERS); })))
+        if ((rc = add_conditional(q.who, s1, h_fused, cudaGraphCondTypeIf, &body)) ||
+            (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_FUSED); })) ||
+            (rc = add_conditional(q.who, s1, h_layers, cudaGraphCondTypeIf, &body)) ||
+            (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_LAYERS); })))
             return rc;
     }
     if (rc != BRL_OK) return rc;
-    void* b[21] = {q.at(q.L.state), q.at(q.L.action), const_cast<void*>(q.table)};
-    for (int t = 0; t < 2; ++t)
-        for (int k = 0; k < 6; ++k) b[3 + 6 * t + k] = q.info[t][k];
-    b[15] = q.at(q.L.state);
-    b[16] = q.at(q.L.obs);
-    b[17] = q.at(q.L.mask);
-    b[18] = q.at(q.L.rewards);
-    b[19] = q.at(q.L.terminated);
-    b[20] = q.at(q.L.player);
-    const BrlParams p = env_params(q, q.n);
-    if ((rc = brl_duplicate_step(s1, b, &p, sizeof(p)))) return rc;  // src/evaluation.py:164
-    k_add_reward<<<(unsigned)((q.n + 255) / 256), 256, 0, s1>>>(q.cum_return, q.at<float4>(q.L.rewards), q.n);
-    if ((rc = check_launch("brl_duplicate_match (cum_return)"))) return rc;
+    if (q.acc) {  // the acting team's masked argmax and update_log_info; free-run: team 2 passes, its forwarded rows unread
+        void* b[7] = {q.logits, q.free_run ? nullptr : q.logits, q.mask, q.player, q.terminated, q.at(q.L.action), q.acc};
+        BrlParams p{};
+        p.n_envs = q.n;
+        p.flags = q.mode == BRL_EVAL_MATCH_SINGLE ? BRL_F_EVAL_INDICATOR_BIDS : 0;
+        if ((rc = brl_eval_act_log(s1, b, &p, sizeof(p)))) return rc;
+    }
+    if ((rc = env_step(q, s1))) return rc;
+    if (q.mode == BRL_EVAL_MATCH_SIMPLE)
+        k_add_actor_reward<<<blocks(q.n), 256, 0, s1>>>(q.cum_return, q.at<float>(q.L.rewards), q.at<int8_t>(q.L.actor), q.n);
+    else if (q.mode == BRL_EVAL_MATCH_SINGLE)
+        k_sum_rewards<<<blocks(q.n), 256, 0, s1>>>(q.cum_return, reinterpret_cast<float4*>(q.rewards_sum), q.at<float4>(q.L.rewards), q.n);
+    else
+        k_add_reward<<<blocks(q.n), 256, 0, s1>>>(q.cum_return, q.at<float4>(q.L.rewards), q.n);
+    if ((rc = launched(q.who, "cum_return"))) return rc;
     if ((rc = model_rows(q, s1))) return rc;
     return control(q, s1, loop);
+}
+
+// brl_evaluate_match's end: the final state's fields and every log_info sum (src/evaluation.py:448-596, :839-1027)
+static int32_t emit_summary(const MatchPlan& q, cudaStream_t s) {
+    void* f[6];
+    for (int k = 0; k < 6; ++k) f[k] = q.at(q.L.fields[k]);
+    const bool single = q.mode == BRL_EVAL_MATCH_SINGLE;
+    void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, single ? f[1] : nullptr, single ? f[2] : nullptr,
+                    single ? f[4] : nullptr, single ? f[5] : nullptr, single ? f[3] : nullptr, f[0], nullptr};
+    BrlParams p = env_params(q, q.n);
+    int32_t rc;
+    if ((rc = brl_state_fields(s, bf, &p, sizeof(p)))) return rc;
+    void* bs[16] = {q.acc, q.cum_return, f[0]};
+    if (single) {  // table A = the final state's fields (no rewards: the sign comes from cum_return), no table B
+        bs[3] = f[1];
+        bs[4] = f[2];
+        bs[5] = f[4];
+        bs[6] = f[5];
+        bs[8] = f[3];
+    } else {       // both Table_infos: last_bid, last_bidder, call_x, call_xx, rewards
+        for (int t = 0; t < 2; ++t) {
+            bs[3 + 6 * t] = q.info[t][2];
+            bs[4 + 6 * t] = q.info[t][3];
+            bs[5 + 6 * t] = q.info[t][4];
+            bs[6 + 6 * t] = q.info[t][5];
+            bs[7 + 6 * t] = q.info[t][1];
+        }
+    }
+    bs[15] = q.sums;
+    BrlParams ps{};
+    ps.n_envs = q.n;
+    return brl_eval_summary(s, bs, &ps, sizeof(ps));
 }
 
 // the whole match on the capturing stream s0 (its own capture, or the caller's)
 static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, cudaStream_t s2) {
     int32_t rc;
     cudaGraphConditionalHandle loop;
-    if ((rc = new_handle(s0, &loop))) return rc;
+    if ((rc = new_handle(q.who, s0, &loop))) return rc;
     const size_t un = (size_t)q.n;
     if (cudaMemsetAsync(q.status, 0, sizeof(int32_t), s0) != cudaSuccess ||
         cudaMemsetAsync(q.at(q.L.ctl), 0, sizeof(int32_t), s0) != cudaSuccess ||
         cudaMemsetAsync(q.cum_return, 0, un * sizeof(float), s0) != cudaSuccess ||
-        cudaMemsetAsync(q.at(q.L.action), 0, un * sizeof(int32_t), s0) != cudaSuccess)  // finished envs keep a (no-op) Pass
-        return check_launch("brl_duplicate_match (memset)");
-    if (q.default_models) k_pair_models<<<(unsigned)((q.n + 255) / 256), 256, 0, s0>>>(q.env_models, q.n);
+        cudaMemsetAsync(q.at(q.L.action), 0, un * sizeof(int32_t), s0) != cudaSuccess ||  // finished envs keep a (no-op) Pass
+        (q.acc && cudaMemsetAsync(q.acc, 0, un * BRL_EVAL_ACC_COLS * sizeof(float), s0) != cudaSuccess) ||
+        (q.logits && cudaMemsetAsync(q.logits, 0, un * BRL_NUM_ACTIONS * sizeof(float), s0) != cudaSuccess) ||
+        (q.rewards_sum && cudaMemsetAsync(q.rewards_sum, 0, un * 16, s0) != cudaSuccess) ||
+        (q.free_run && cudaMemsetAsync(q.env_models, 0, un * 8, s0) != cudaSuccess))  // free-run: net 0 forwards every row
+        return launched(q.who, "memset");
+    if (q.default_models) k_pair_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.n);
     // src/evaluation.py:93-95: the envs from the given keys, observation in bf16 (what the forward reads)
-    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.at(q.L.state), q.at(q.L.obs), q.at(q.L.mask),
-                   q.at(q.L.rewards), q.at(q.L.terminated), q.at(q.L.player)};
+    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
+                   q.player};
     BrlParams p = env_params(q, q.n);
     if ((rc = brl_init(s0, bi, &p, sizeof(p)))) return rc;
-    // :97-112 Table_info A = B = the init state's terminated, rewards, last_bid, last_bidder, call_x, call_xx
-    void* bf[12] = {q.at(q.L.state), nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
-    if ((rc = brl_state_fields(s0, bf, &p, sizeof(p)))) return rc;
-    const size_t bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
-    if (cudaMemcpyAsync(q.info[0][0], q.at(q.L.terminated), bytes[0], cudaMemcpyDeviceToDevice, s0) != cudaSuccess ||
-        cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-        return check_launch("brl_duplicate_match (Table_info)");
-    for (int k = 0; k < 6; ++k)
-        if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-            return check_launch("brl_duplicate_match (Table_info)");
+    if (q.mode == BRL_EVAL_MATCH_SIMPLE) {
+        k_actor_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player), q.n);
+        if ((rc = launched(q.who, "actor"))) return rc;
+    }
+    if (q.mode == 0 || q.mode == BRL_EVAL_MATCH_DUPLICATE) {
+        // :97-112 Table_info A = B = the init state's terminated, rewards, last_bid, last_bidder, call_x, call_xx
+        void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
+        if ((rc = brl_state_fields(s0, bf, &p, sizeof(p)))) return rc;
+        const size_t bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
+        if (cudaMemcpyAsync(q.info[0][0], q.terminated, bytes[0], cudaMemcpyDeviceToDevice, s0) != cudaSuccess ||
+            cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
+            return launched(q.who, "Table_info");
+        for (int k = 0; k < 6; ++k)
+            if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
+                return launched(q.who, "Table_info");
+    }
     if ((rc = model_rows(q, s0)) || (rc = control(q, s0, loop))) return rc;
     cudaGraph_t body;
-    if ((rc = add_conditional(s0, loop, cudaGraphCondTypeWhile, &body)) ||
-        (rc = capture_into(body, s1, [&](cudaStream_t s) { return emit_body(q, s, s2, loop); })))
+    if ((rc = add_conditional(q.who, s0, loop, cudaGraphCondTypeWhile, &body)) ||
+        (rc = capture_into(q.who, body, s1, [&](cudaStream_t s) { return emit_body(q, s, s2, loop); })))
         return rc;
+    if (q.mode == BRL_EVAL_MATCH_SIMPLE) return BRL_OK;  // the output is R itself
+    if (q.mode != 0) return emit_summary(q, s0);
     // :199-201 the match sums, per range
     if (q.ranges) {
         void* bs[3] = {q.cum_return, const_cast<int64_t*>(q.ranges), q.sums};
@@ -306,14 +435,87 @@ static MatchCache& cache() {
 }
 constexpr size_t kMaxCachedGraphs = 16;
 
-static int32_t capture_streams(cudaStream_t** out) {
+static int32_t capture_streams(const char* who, cudaStream_t** out) {
     cudaStream_t* s = cache().streams[device_slot()];
     for (int k = 0; k < 3; ++k)
         if (s[k] == nullptr && cudaStreamCreateWithFlags(&s[k], cudaStreamNonBlocking) != cudaSuccess)
-            return check_launch("brl_duplicate_match (capture stream)");
+            return launched(who, "capture stream");
     *out = s;
     return BRL_OK;
 }
+
+// run plan q on `stream`: into the caller's capture when the stream is being captured, else by (building and caching, keyed by
+// the op's params and its n_buffers buffer addresses, then) launching the match's graph
+static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p, void** b, int n_buffers) {
+    int32_t rc;
+    cudaStreamCaptureStatus st;
+    if (cudaStreamIsCapturing(s, &st) != cudaSuccess) return launched(q.who, "capture status");
+    MatchCache& c = cache();
+    std::lock_guard<std::mutex> lock(c.mu);
+    cudaStream_t* side = nullptr;
+    if ((rc = warm_policy_grouped_dev(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(q.who, &side))) return rc;
+    if (st == cudaStreamCaptureStatusActive) {  // the caller's capture: the nodes go there
+        if ((rc = emit_match(q, s, side[1], side[2]))) return rc;
+        return check_launch(q.who);
+    }
+    if (st != cudaStreamCaptureStatusNone) return fail(BRL_E_LAUNCH, "%s: the stream's capture was invalidated", q.who);
+    int dev = 0;
+    cudaGetDevice(&dev);
+    std::string key(reinterpret_cast<const char*>(&dev), sizeof(dev));
+    key.append(reinterpret_cast<const char*>(p), sizeof(*p));
+    key.append(reinterpret_cast<const char*>(b), n_buffers * sizeof(void*));
+    auto it = c.exec.find(key);
+    if (it == c.exec.end()) {
+        if (cudaStreamBeginCapture(side[0], cudaStreamCaptureModeRelaxed) != cudaSuccess) return launch_error(q.who, "capture");
+        rc = emit_match(q, side[0], side[1], side[2]);
+        cudaGraph_t g = nullptr;
+        const cudaError_t end = cudaStreamEndCapture(side[0], &g);
+        cudaGraphExec_t exec = nullptr;
+        if (rc == BRL_OK && (end != cudaSuccess || cudaGraphInstantiate(&exec, g, 0) != cudaSuccess))
+            rc = launch_error(q.who, "instantiate");
+        if (g != nullptr) cudaGraphDestroy(g);
+        if (rc != BRL_OK) return rc;
+        if (c.exec.size() >= kMaxCachedGraphs) {  // evict the least recently used (a graph still running is freed when it ends)
+            auto lru = c.exec.begin();
+            for (auto e = c.exec.begin(); e != c.exec.end(); ++e)
+                if (e->second.second < lru->second.second) lru = e;
+            cudaGraphExecDestroy(lru->second.first);
+            c.exec.erase(lru);
+        }
+        it = c.exec.emplace(key, std::make_pair(exec, (uint64_t)0)).first;
+        ++c.builds;
+    }
+    it->second.second = ++c.clock;
+    if (cudaGraphLaunch(it->second.first, s) != cudaSuccess) return launched(q.who, "launch");
+    return check_launch(q.who);
+}
+
+// the plan's fields every mode shares; the env buffers and Table_infos start in the scratch
+static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_t M, void* scratch) {
+    MatchPlan q{};
+    q.who = who;
+    q.mode = mode;
+    q.n = p->n_envs;
+    q.M = (int)M;
+    q.cap = brl_model_rows_capacity(q.n, M);
+    q.n_deals = p->n_deals;
+    q.flags = p->flags;
+    q.illegal_penalty = p->illegal_penalty;
+    q.illegal_bonus = p->illegal_bonus;
+    q.scratch = static_cast<unsigned char*>(scratch);
+    q.L = match_layout(q.n, M, mode);
+    for (int t = 0; t < 2; ++t)
+        for (int k = 0; k < 6; ++k) q.info[t][k] = q.at(q.L.info[t][k]);
+    q.state = q.at(q.L.state);
+    q.obs = q.at(q.L.obs);
+    q.mask = q.at(q.L.mask);
+    q.terminated = q.at(q.L.terminated);
+    q.player = q.at(q.L.player);
+    q.env_models = q.at<int32_t>(q.L.env_models);
+    return q;
+}
+
+static bool misaligned(const void* ptr, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(ptr) & (bytes - 1)) != 0; }
 
 }  // namespace brl
 
@@ -359,70 +561,91 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     if (given && ((reinterpret_cast<uintptr_t>(b[10]) | reinterpret_cast<uintptr_t>(b[16])) & 15u))
         return fail(BRL_E_BUFFER, "brl_duplicate_match: Table_info rewards are not 16-byte aligned");
 
-    MatchPlan q{};
-    q.n = p->n_envs;
-    q.M = (int)M;
+    MatchPlan q = base_plan("brl_duplicate_match", 0, p, M, b[5]);
     q.P = P;
-    q.cap = brl_model_rows_capacity(q.n, M);
-    q.n_deals = p->n_deals;
-    q.flags = p->flags;
-    q.illegal_penalty = p->illegal_penalty;
-    q.illegal_bonus = p->illegal_bonus;
     q.keys = b[0];
     q.table = b[1];
     q.pool = static_cast<const unsigned char*>(b[2]);
     q.ranges = static_cast<const int64_t*>(b[4]);
-    q.scratch = static_cast<unsigned char*>(b[5]);
     q.cum_return = static_cast<float*>(b[6]);
     q.sums = static_cast<double*>(b[7]);
     q.status = static_cast<int32_t*>(b[8]);
-    q.L = match_layout(q.n, M);
-    for (int t = 0; t < 2; ++t)
-        for (int k = 0; k < 6; ++k) q.info[t][k] = given ? b[9 + 6 * t + k] : q.at(q.L.info[t][k]);
+    if (given)
+        for (int t = 0; t < 2; ++t)
+            for (int k = 0; k < 6; ++k) q.info[t][k] = b[9 + 6 * t + k];
     q.default_models = b[3] == nullptr;
-    q.env_models = q.default_models ? q.at<int32_t>(q.L.env_models) : static_cast<int32_t*>(b[3]);
+    if (!q.default_models) q.env_models = static_cast<int32_t*>(b[3]);
+    return run_match(q, (cudaStream_t)stream, p, b, 21);
+}
 
-    cudaStream_t s = (cudaStream_t)stream;
-    cudaStreamCaptureStatus st;
-    if (cudaStreamIsCapturing(s, &st) != cudaSuccess) return check_launch("brl_duplicate_match (capture status)");
-    MatchCache& c = cache();
-    std::lock_guard<std::mutex> lock(c.mu);
-    cudaStream_t* side = nullptr;
-    if ((rc = warm_policy_grouped_dev(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(&side))) return rc;
-    if (st == cudaStreamCaptureStatusActive) {  // the caller's capture: the nodes go there
-        if ((rc = emit_match(q, s, side[1], side[2]))) return rc;
-        return check_launch("brl_duplicate_match");
+int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode) {
+    if (n_envs <= 0 || mode < BRL_EVAL_MATCH_DUPLICATE || mode > BRL_EVAL_MATCH_SIMPLE) return 0;
+    return (int64_t)match_layout(n_envs, 2, (int)mode).total;
+}
+
+int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    const int mode = BRL_EVAL_MATCH_MODE(p->flags);
+    const bool free_run = (p->flags & BRL_F_EVAL_FREE_RUN) != 0, full = mode != BRL_EVAL_MATCH_SIMPLE;
+    if (mode < BRL_EVAL_MATCH_DUPLICATE || mode > BRL_EVAL_MATCH_SIMPLE)
+        return fail(BRL_E_OPAQUE, "brl_evaluate_match: flags name no mode (BRL_F_EVAL_MATCH(BRL_EVAL_MATCH_*))");
+    if (free_run && !full) return fail(BRL_E_OPAQUE, "brl_evaluate_match: BRL_F_EVAL_FREE_RUN is a mode of the full-statistics evaluation");
+    if (p->n_envs > INT32_MAX / 2) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_envs too large");
+    if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_deals must be > 0");
+    if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_evaluate_match: sampling is not supported (argmax only)");
+    BRL_REQUIRE(b[0], "keys");
+    BRL_REQUIRE(b[1], "deal_table");
+    BRL_REQUIRE(b[2], "pool");
+    BRL_REQUIRE(b[3], "scratch");
+    if (b[4] == nullptr || misaligned(b[4], 4)) return fail(BRL_E_BUFFER, "brl_evaluate_match: cum_return is NULL or misaligned");
+    if (full && (b[5] == nullptr || misaligned(b[5], 4))) return fail(BRL_E_BUFFER, "brl_evaluate_match: acc is NULL or misaligned");
+    if (full && (b[6] == nullptr || misaligned(b[6], 8))) return fail(BRL_E_BUFFER, "brl_evaluate_match: sums is NULL or misaligned");
+    if (b[7] == nullptr || misaligned(b[7], 4)) return fail(BRL_E_BUFFER, "brl_evaluate_match: status is NULL or misaligned");
+    int tables = 0, finals = 0;
+    for (int k = 8; k < 20; ++k) tables += b[k] != nullptr;
+    for (int k = 20; k < 26; ++k) finals += b[k] != nullptr;
+    if (mode == BRL_EVAL_MATCH_DUPLICATE) {
+        if (tables != 0 && tables != 12) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all twelve Table_info buffers [8..19] or none");
+        if (tables && (misaligned(b[9], 16) || misaligned(b[15], 16)))
+            return fail(BRL_E_BUFFER, "brl_evaluate_match: Table_info rewards are not 16-byte aligned");
     }
-    if (st != cudaStreamCaptureStatusNone) return fail(BRL_E_LAUNCH, "brl_duplicate_match: the stream's capture was invalidated");
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::string key(reinterpret_cast<const char*>(&dev), sizeof(dev));
-    key.append(reinterpret_cast<const char*>(p), sizeof(*p));
-    key.append(reinterpret_cast<const char*>(b), 21 * sizeof(void*));
-    auto it = c.exec.find(key);
-    if (it == c.exec.end()) {
-        if (cudaStreamBeginCapture(side[0], cudaStreamCaptureModeRelaxed) != cudaSuccess) return launch_error("brl_duplicate_match (capture)");
-        rc = emit_match(q, side[0], side[1], side[2]);
-        cudaGraph_t g = nullptr;
-        const cudaError_t end = cudaStreamEndCapture(side[0], &g);
-        cudaGraphExec_t exec = nullptr;
-        if (rc == BRL_OK && (end != cudaSuccess || cudaGraphInstantiate(&exec, g, 0) != cudaSuccess))
-            rc = launch_error("brl_duplicate_match (instantiate)");
-        if (g != nullptr) cudaGraphDestroy(g);
-        if (rc != BRL_OK) return rc;
-        if (c.exec.size() >= kMaxCachedGraphs) {  // evict the least recently used (a graph still running is freed when it ends)
-            auto lru = c.exec.begin();
-            for (auto e = c.exec.begin(); e != c.exec.end(); ++e)
-                if (e->second.second < lru->second.second) lru = e;
-            cudaGraphExecDestroy(lru->second.first);
-            c.exec.erase(lru);
+    if (mode == BRL_EVAL_MATCH_SINGLE) {
+        if (finals != 0 && finals != 6) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all six final-state buffers [20..25] or none");
+        if (finals && (misaligned(b[20], 16) || misaligned(b[21], 16) || misaligned(b[22], 2) || misaligned(b[23], 16)))
+            return fail(BRL_E_BUFFER, "brl_evaluate_match: the final state, observation or rewards are not 16-byte aligned (mask: 2)");
+    }
+
+    MatchPlan q = base_plan("brl_evaluate_match", mode, p, 2, b[3]);
+    q.free_run = free_run;
+    q.keys = b[0];
+    q.table = b[1];
+    q.pool = static_cast<const unsigned char*>(b[2]);
+    q.cum_return = static_cast<float*>(b[4]);
+    q.status = static_cast<int32_t*>(b[7]);
+    q.default_models = mode != BRL_EVAL_MATCH_SIMPLE && !free_run;
+    if (full) {
+        q.acc = static_cast<float*>(b[5]);
+        q.sums = static_cast<double*>(b[6]);
+        q.logits = q.at<float>(q.L.logits);
+    }
+    if (mode == BRL_EVAL_MATCH_DUPLICATE && tables)
+        for (int t = 0; t < 2; ++t)
+            for (int k = 0; k < 6; ++k) q.info[t][k] = b[8 + 6 * t + k];
+    if (mode == BRL_EVAL_MATCH_SINGLE) {
+        q.rewards_sum = q.at<float>(q.L.rewards_sum);
+        if (finals) {
+            q.state = b[20];
+            q.obs = b[21];
+            q.mask = b[22];
+            q.rewards_sum = static_cast<float*>(b[23]);
+            q.terminated = b[24];
+            q.player = b[25];
         }
-        it = c.exec.emplace(key, std::make_pair(exec, (uint64_t)0)).first;
-        ++c.builds;
     }
-    it->second.second = ++c.clock;
-    if (cudaGraphLaunch(it->second.first, s) != cudaSuccess) return check_launch("brl_duplicate_match (launch)");
-    return check_launch("brl_duplicate_match");
+    return run_match(q, (cudaStream_t)stream, p, b, 26);
 }
 
 }  // extern "C"

@@ -1171,13 +1171,14 @@ int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t
 
 namespace brl {
 
-// ---- the grouped forward of brl_duplicate_match's device loop (brl_match.cu) ------------------------------------------------
+// ---- the grouped forward of the device loops of brl_duplicate_match / brl_evaluate_match (brl_match.cu) ---------------------
 // brl_policy_act_grouped with the padded row count in device memory (`n_rows` = brl_model_rows' offsets[M]): the gather, the
 // launches and their tensor maps are sized for `capacity` rows, and the DEVCOUNT kernels stop at the count.  The caller picks the
-// path: `flags` holds BRL_F_TUNE_MLP_LAYERS or BRL_F_TUNE_MLP_FUSED (and BRL_F_MLP_BF16 for the single-product mode).
+// path: `flags` holds BRL_F_TUNE_MLP_LAYERS or BRL_F_TUNE_MLP_FUSED (and BRL_F_MLP_BF16 for the single-product mode).  `logits`
+// (f32[n, 38] or NULL): the listed rows' logits, written by env as brl_policy_act_grouped's buffer [7].
 int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
                                   const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
-                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows) {
+                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits) {
     BrlParams p{};
     p.n_envs = capacity;
     p.flags = flags;
@@ -1191,14 +1192,14 @@ int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacit
     act.action = action;
     act.row_index = rows;
     const PoolArgs pa{block_model, brl_mlp_pool_stride(), n_models, act, n_rows};
-    return mlp_forward_impl<true, true>("brl_duplicate_match", s, &p, gathered, pool, reinterpret_cast<__nv_bfloat16*>(scratch),
-                                        nullptr, nullptr, act, &pa);
+    return mlp_forward_impl<true, true>("grouped forward (device count)", s, &p, gathered, pool, reinterpret_cast<__nv_bfloat16*>(scratch),
+                                        logits, nullptr, act, &pa);
 }
 
 // everything launch_policy_grouped_dev sets up once per device -- the driver's tensor-map entry point, the kernels'
 // shared-memory attributes, the fused kernel's co-resident pair count -- done before a stream capture begins
 int32_t warm_policy_grouped_dev(bool split) {
-    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_duplicate_match: cuTensorMapEncodeTiled not available from the driver");
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "device match loop: cuTensorMapEncodeTiled not available from the driver");
     int32_t rc;
     if (split) {
         if ((rc = layer_attr<128, false, true, false, true, true>()) || (rc = layer_attr<128, true, true, false, true, true>()) ||

@@ -75,6 +75,7 @@
     X(brl_policy_act_grouped, "iisixiix") \
     X(brl_match_stats_ranges, "iix") \
     X(brl_duplicate_match, "iiiiisoxooooooooooooo") \
+    X(brl_evaluate_match, "iiisooxooooooooooooooooooo") \
     /* end */
 
 namespace {

@@ -1,5 +1,6 @@
 """Evaluation loops of src/evaluation.py: `make_simple_duplicate_evaluate` (69-204, the
-eval.py path and the league probe) and `make_simple_evaluate` (11-66)."""
+eval.py path and the league probe), `make_simple_evaluate` (11-66) and `make_evaluate` (207-1032),
+each as a host loop and as a device loop (one brl_duplicate_match / brl_evaluate_match call)."""
 from __future__ import annotations
 
 import torch
@@ -304,11 +305,11 @@ class _MatchBuffers:
                             illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
 
 
-def _check_match_status(status: int) -> None:
+def _check_match_status(status: int, op: str = "brl_duplicate_match") -> None:
     if status == ops._lib.MATCH_BAD_MODEL:
-        raise ops._lib.BrlError("brl_duplicate_match: an acting net id is outside [0, M)")
+        raise ops._lib.BrlError(f"{op}: an acting net id is outside [0, M)")
     if status != ops._lib.MATCH_OK:
-        raise ops._lib.BrlError(f"brl_duplicate_match: envs still live after {ops._lib.MATCH_MAX_STEPS} steps (status {status})")
+        raise ops._lib.BrlError(f"{op}: envs still live after {ops._lib.MATCH_MAX_STEPS} steps (status {status})")
 
 
 def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_envs, env_offset: int = 0, *, tune: int = 0):
@@ -525,3 +526,124 @@ def make_evaluate_log(log_info):
                 log[f"eval/{name}/{number}{suit}"] = vec[index]
                 index += 1
     return log
+
+
+# ---- the device-loop twins of make_evaluate / make_simple_evaluate: one brl_evaluate_match call each (ppo.py:365-374) ----------
+class _EvalBuffers:
+    """Fixed-address inputs and outputs of brl_evaluate_match for one shape and mode (as _MatchBuffers: repeated calls
+    relaunch the op's cached graph)."""
+
+    def __init__(self, n: int, mode: int, dev):
+        L = ops._lib
+        self.mode = mode
+        self.keys = torch.empty(n, dtype=torch.int64, device=dev)
+        self.pool = torch.zeros((2, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
+        self.scratch = torch.empty(ops.evaluate_match_scratch_bytes(n, mode), dtype=torch.uint8, device=dev)
+        self.cum_return = torch.empty(n, dtype=torch.float32, device=dev)
+        self.status = torch.zeros(1, dtype=torch.int32, device=dev)
+        full = mode != L.EVAL_MATCH_SIMPLE
+        self.acc = torch.empty((n, L.EVAL_ACC_COLS), dtype=torch.float32, device=dev) if full else None
+        self.sums = torch.zeros(L.load().brl_eval_num_sums(), dtype=torch.float64, device=dev) if full else None
+        dup = mode == L.EVAL_MATCH_DUPLICATE
+        self.tables = (ops.TableInfoBuffers(n, dev), ops.TableInfoBuffers(n, dev)) if dup else (None, None)
+        single = mode == L.EVAL_MATCH_SINGLE
+        self.final_state = ops.new_state(n, dev) if single else None
+        self.final = ops.EnvOutputs(n, dev, torch.bfloat16) if single else None
+
+    def play(self, eval_env, single_bf16: bool, free_run: bool, tune: int):
+        if self.sums is not None:
+            self.sums.zero_()
+        ops.evaluate_match(self.keys, eval_env.table, self.pool, self.scratch, self.cum_return, self.status, mode=self.mode,
+                           acc=self.acc, sums=self.sums, table_a=self.tables[0], table_b=self.tables[1],
+                           final_state=self.final_state, final=self.final, free_run=free_run, single_bf16=single_bf16, tune=tune,
+                           illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
+
+
+def _one_precision(actor_forward_pass, opp_forward_pass) -> bool:
+    """the single_bf16 flag of a pool holding both nets (it holds one architecture and one precision)"""
+    if actor_forward_pass.precision != opp_forward_pass.precision:
+        raise ValueError("the device evaluation runs both teams in one precision")
+    return actor_forward_pass.precision == "tc-bf16"
+
+
+def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_activation, team2_model_type, team2_model_path,
+                         num_eval_envs, game_mode, duplicate=False, team2_params=None, env_offset: int = 0, *, tune: int = 0):
+    """make_evaluate (src/evaluation.py:207-1032) with the whole loop in one brl_evaluate_match call: the loop runs on the
+    device (a CUDA graph WHILE node), so an evaluation costs one launch and one host read of its statistics.  Same contract --
+    `duplicate_evaluate(actor_params, rng_key) -> (log_info, table_a_info, table_b_info)` or `evaluate(actor_params, rng_key) ->
+    (state, log_info)`, same key split and keys, `env_offset` sharding, one all-reduce of the statistics over the ranks -- and
+    the same per-env results.  In "free-run" team 2's rows are forwarded by the actor's net and not read (brl_evaluate_match).
+    `trace` needs per-step host copies: use make_evaluate for it.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path.
+    The returned function's `buffers` hold the last call's per-env `acc` rows and `cum_return`."""
+    L = ops._lib
+    actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
+    opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
+    if game_mode == "competitive":
+        opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
+    elif game_mode == "free-run":
+        opp_params = None
+    else:
+        raise ValueError(game_mode)
+    single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
+    n, dev = num_eval_envs, eval_env.device
+    bufs = _EvalBuffers(n, L.EVAL_MATCH_DUPLICATE if duplicate else L.EVAL_MATCH_SINGLE, dev)
+    blob_bytes = L.load().brl_mlp_packed_bytes()
+
+    def play(actor_params, rng_key):
+        rng_key, sub_key = brandom.split(rng_key)
+        bufs.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))
+        actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
+        if opp_params is not None:
+            opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
+        bufs.play(eval_env, single_bf16, opp_params is None, tune)
+        sums = bufs.sums.clone()
+        bdist.allreduce_sums(sums)
+        host = torch.cat((sums, bufs.status.to(torch.float64))).cpu().numpy()
+        _check_match_status(int(host[-1]), "brl_evaluate_match")
+        return host[:-1]
+
+    def evaluate(actor_params, rng_key):
+        sums = play(actor_params, rng_key)
+        from .env import State
+        out = ops.EnvOutputs(n, dev, torch.bfloat16)
+        for k in ops.EnvOutputs.__slots__:
+            getattr(out, k).copy_(getattr(bufs.final, k))
+        return State(eval_env, bufs.final_state.clone(), out), _log_info_from_sums(sums, duplicate=False)
+
+    def duplicate_evaluate(actor_params, rng_key):
+        sums = play(actor_params, rng_key)
+        infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
+                            t.call_xx.clone()) for t in bufs.tables]
+        return _log_info_from_sums(sums, duplicate=True), infos[0], infos[1]
+
+    fn = duplicate_evaluate if duplicate else evaluate
+    fn.buffers = bufs
+    return fn
+
+
+def make_device_simple_evaluate(eval_env, team1_activation, team1_model_type, team2_activation, team2_model_type,
+                                team2_model_path, num_eval_envs, team2_params=None, *, tune: int = 0):
+    """make_simple_evaluate (src/evaluation.py:11-66) as one brl_evaluate_match call: the same keys and per-env returns R, and
+    `simple_evaluate(actor_params, rng) -> R.mean()`.  Every decision is an argmax and the net acting is fixed per seat, so the
+    device loop takes one env step per iteration and forwards each live env through the one net that acts there, where the
+    host loop forwards both nets over every env until the last auction ends.  `trace` needs per-step host copies: use
+    make_simple_evaluate for it.  The returned function's `buffers.cum_return` holds the last call's R."""
+    L = ops._lib
+    actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
+    opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
+    opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
+    single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
+    bufs = _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device)
+    blob_bytes = L.load().brl_mlp_packed_bytes()
+
+    def simple_evaluate(actor_params, rng):
+        rng_key, sub_key = brandom.split(rng)
+        bufs.keys.copy_(eval_env.make_keys(sub_key, num_eval_envs))
+        actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
+        opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
+        bufs.play(eval_env, single_bf16, False, tune)
+        _check_match_status(int(bufs.status[0]), "brl_evaluate_match")
+        return bufs.cum_return.mean()
+
+    simple_evaluate.buffers = bufs
+    return simple_evaluate

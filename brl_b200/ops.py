@@ -609,3 +609,51 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
                                   _ptr(cum_return), _ptr(sums), _ptr(status)] + infos,
           _params(n, k_steps=M, step=P, n_deals=table.shape[0], flags=(F_MLP_BF16 if single_bf16 else 0) | tune,
                   illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))
+
+
+# ---- a whole evaluation as one call (ppo.py:365-374; src/evaluation.py:11-66, 207-1032) -----------------------------------
+def evaluate_match_scratch_bytes(n_envs: int, mode: int) -> int:
+    return _size_query("brl_evaluate_match_scratch_bytes", n_envs, mode)
+
+
+def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, cum_return: torch.Tensor,
+                   status: torch.Tensor, *, mode: int, acc: Optional[torch.Tensor] = None, sums: Optional[torch.Tensor] = None,
+                   table_a: Optional[TableInfoBuffers] = None, table_b: Optional[TableInfoBuffers] = None,
+                   final_state: Optional[torch.Tensor] = None, final: Optional[EnvOutputs] = None, free_run: bool = False,
+                   single_bf16: bool = False, tune: int = 0, illegal_penalty: float = -1.0, illegal_bonus: float = 1.0) -> None:
+    """Play a whole evaluation (make_evaluate's duplicate_evaluate / evaluate, or make_simple_evaluate) for every env of `keys`
+    in one call, with the loop on the device.  `pool` u8[2, mlp_pool_stride()]: net 0 is team 1 / the actor, net 1 team 2 / the
+    opponent (not read with free_run).  `mode` = _lib.EVAL_MATCH_*:
+      DUPLICATE / SINGLE: writes cum_return f32[n] and acc f32[n, EVAL_ACC_COLS], adds brl_eval_summary's partial sums to `sums`
+        (f64[brl_eval_num_sums()]); DUPLICATE writes the final Table_infos when given, SINGLE the final state (`final_state`
+        int32[5, n, 4], `final` with a bf16 observation; its rewards = the summed step rewards) when given;
+      SIMPLE: cum_return = R, the per-env return of the player to act at the start.
+    `status` (int32[1], _lib.MATCH_*) is written too; nothing is read back to the host."""
+    n = int(keys.shape[0])
+    if mode not in (_lib.EVAL_MATCH_DUPLICATE, _lib.EVAL_MATCH_SINGLE, _lib.EVAL_MATCH_SIMPLE):
+        raise _lib.BrlError(f"evaluate_match: unknown mode {mode}")
+    full = mode != _lib.EVAL_MATCH_SIMPLE
+    if free_run and not full:
+        raise _lib.BrlError("evaluate_match: free_run is a mode of the full-statistics evaluation")
+    if pool.dim() != 2 or pool.dtype != torch.uint8 or tuple(pool.shape) != (2, mlp_pool_stride()):
+        raise _lib.BrlError("evaluate_match: pool must be u8[2, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    if cum_return.dtype != torch.float32 or status.dtype != torch.int32:
+        raise _lib.BrlError("evaluate_match: cum_return must be float32 and status int32")
+    if full:
+        if acc is None or sums is None or acc.dtype != torch.float32 or tuple(acc.shape) != (n, _lib.EVAL_ACC_COLS) or \
+                sums.dtype != torch.float64 or sums.numel() != _lib.load().brl_eval_num_sums():
+            raise _lib.BrlError("evaluate_match: full statistics need acc float32[n, 76] and sums float64[239]")
+    if scratch.numel() < evaluate_match_scratch_bytes(n, mode):
+        raise _lib.BrlError("evaluate_match: scratch too small (ops.evaluate_match_scratch_bytes)")
+    if (table_a is None) != (table_b is None):
+        raise _lib.BrlError("evaluate_match: give both Table_info outputs or neither")
+    if (final_state is None) != (final is None):
+        raise _lib.BrlError("evaluate_match: give the final state and its outputs together or neither")
+    if final is not None and final.observation.dtype != torch.bfloat16:
+        raise _lib.BrlError("evaluate_match: the final observation is bf16")
+    infos = table_a.ptrs() + table_b.ptrs() if table_a is not None else [None] * 12
+    finals = [_ptr(final_state)] + final.ptrs() if final is not None else [None] * 6
+    flags = _lib.f_eval_match(mode) | (_lib.F_EVAL_FREE_RUN if free_run else 0) | (F_MLP_BF16 if single_bf16 else 0) | tune
+    _call("brl_evaluate_match", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(scratch), _ptr(cum_return), _ptr(acc), _ptr(sums),
+                                 _ptr(status)] + infos + finals,
+          _params(n, n_deals=table.shape[0], flags=flags, illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))

@@ -22,7 +22,8 @@ import torch
 from . import deals as _deals
 from . import random as brandom
 from .env import BridgeBidding
-from .evaluation import make_evaluate, make_evaluate_log, make_simple_duplicate_evaluate, make_simple_evaluate
+from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_simple_evaluate, make_evaluate,
+                         make_evaluate_log, make_simple_duplicate_evaluate, make_simple_evaluate)
 from .gae import make_calc_gae
 from .models import LAYERS, init_params, load_params, make_forward_pass
 from .optim import make_optimizer
@@ -44,7 +45,10 @@ def default_config() -> dict:
         num_prioritized_envs=100, gamma=1.0, gae_lambda=0.95, clip_eps=0.2, ent_coef=0.001, vf_coef=0.5,
         value_clipping=True, global_gradient_clipping=True, anneal_lr=False, reward_scaling=False, max_grad_norm=0.5,
         reward_scale=7600.0, actor_illegal_action_mask=True, actor_illegal_action_penalty=False,
-        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0)
+        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0,
+        # not in PPOConfig: run the three evaluations of every iteration (train/score, eval/*, the imp_opp / PFSP probes) as
+        # device loops, one brl_evaluate_match / brl_duplicate_match call each, with the same results
+        device_eval=False)
 
 
 def params_to_host(params) -> dict:
@@ -62,6 +66,23 @@ def pfsp_probabilities(imp_list: np.ndarray, prior_t: float) -> np.ndarray:
     x = -np.asarray(imp_list, dtype=np.float64)
     e = np.exp((x - x.max()) / prior_t)
     return e / e.sum()
+
+
+def make_evaluators(config: dict, eval_env, eval_opp_params):
+    """The three evaluators of every iteration (ppo.py:252-283): (train/score vs eval_opp, the imp_opp / PFSP duplicate probe,
+    the eval/* duplicate statistics) -- the host loops, or with config["device_eval"] their device-loop twins."""
+    act, mt = config["actor_activation"], config["actor_model_type"]
+    opp_act, opp_mt = config["eval_opp_activation"], config["eval_opp_model_type"]
+    if config["device_eval"]:
+        return (make_device_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"],
+                                            team2_params=eval_opp_params),
+                make_device_duplicate_evaluate(eval_env, act, mt, config["num_prioritized_envs"]),
+                make_device_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"],
+                                     duplicate=True, team2_params=eval_opp_params))
+    return (make_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], team2_params=eval_opp_params),
+            make_simple_duplicate_evaluate(eval_env, act, mt, act, mt, config["num_prioritized_envs"]),
+            make_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"], duplicate=True,
+                          team2_params=eval_opp_params))
 
 
 def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=None, device="cuda",
@@ -107,16 +128,7 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
     if eval_opp_params is None:
         eval_opp_params = (load_params(config["eval_opp_model_path"], dev) if config["eval_opp_model_path"]
                            else init_params(12345, dev))
-    simple_evaluate = make_simple_evaluate(eval_env, config["actor_activation"], config["actor_model_type"],
-                                           config["eval_opp_activation"], config["eval_opp_model_type"], None,
-                                           config["num_eval_envs"], team2_params=eval_opp_params)
-    simple_duplicate_evaluate = make_simple_duplicate_evaluate(eval_env, config["actor_activation"], config["actor_model_type"],
-                                                               config["actor_activation"], config["actor_model_type"],
-                                                               config["num_prioritized_envs"])
-    duplicate_evaluate = make_evaluate(eval_env, config["actor_activation"], config["actor_model_type"],
-                                       config["eval_opp_activation"], config["eval_opp_model_type"], None,
-                                       config["num_eval_envs"], config["game_mode"], duplicate=True,
-                                       team2_params=eval_opp_params)
+    simple_evaluate, simple_duplicate_evaluate, duplicate_evaluate = make_evaluators(config, eval_env, eval_opp_params)
 
     opp_forward_pass = make_fp(config["opp_activation"], config["opp_model_type"])
     envs = [BridgeBidding(table=t, device=dev) for t in tables]                                   # ppo.py:296-303

@@ -66,6 +66,9 @@
  *   brl_match_stats_ranges  brl_match_stats of every match of a league chunk   src/evaluation.py:199-201
  *   brl_duplicate_match   jax.jit(make_simple_duplicate_evaluate(...)) as one call: init, Table_info, the whole
  *                         lax.while_loop and the match sums   eval.py:53 ; src/evaluation.py:69-204
+ *   brl_evaluate_match    jax.jit of make_evaluate's duplicate_evaluate / evaluate or of make_simple_evaluate as one call:
+ *                         init, the whole lax.while_loop with the step log, and the log_info sums (or the actor's returns)
+ *                         ppo.py:365-374 ; src/evaluation.py:11-66, 207-1032
  */
 #ifndef BRL_B200_H
 #define BRL_B200_H
@@ -329,6 +332,45 @@ int64_t brl_duplicate_match_scratch_bytes(int64_t n_envs, int64_t n_models);
 long long brl_duplicate_match_graph_builds(void);
 int32_t brl_duplicate_match(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- a whole evaluation as one call (ppo.py:365-374; src/evaluation.py:11-66, 207-1032) ----------------------------------
+ * brl_duplicate_match's device loop (WHILE node, control kernel, path kernel and IF nodes, graph cache, adding to a caller's
+ * capture, BRL_MATCH_* status and bound) for the other evaluators of ppo.train.  The pool holds two nets: net 0 is team 1 /
+ * the actor, net 1 team 2 / the opponent.  The mode is flags bits 27-28 (BRL_F_EVAL_MATCH(m)):
+ *   BRL_EVAL_MATCH_DUPLICATE  make_evaluate(duplicate=True)'s duplicate_evaluate (:615-1027): brl_init (:617-619) ->
+ *       Table_info A = B (:621-636) -> while any env is live { brl_model_rows -> grouped forward with the logits by env ->
+ *       brl_eval_act_log (:650-745) -> brl_duplicate_step (:772-774) -> cum_return += rewards[:, 0] (:775-777) } ->
+ *       brl_state_fields (step_count) -> brl_eval_summary with both Table_infos into sums (:839-1027).
+ *   BRL_EVAL_MATCH_SINGLE  make_evaluate(duplicate=False)'s evaluate (:256-596): the same loop with brl_step (no auto-reset,
+ *       :406) and rewards_sum += rewards, cum_return += rewards[:, 0] (:407-411); brl_eval_summary takes the final state's
+ *       fields (:448-596); BRL_F_EVAL_INDICATOR_BIDS is implied (:345-354).
+ *   BRL_EVAL_MATCH_SIMPLE  make_simple_evaluate (:11-66): every decision is an argmax and the net acting is fixed per seat, so
+ *       the quad step (src/utils.py:133-202) is one env step per iteration: net 0 decides for the team of the env's INITIAL
+ *       current_player, net 1 for the other team; R[i] += rewards[i, initial player] per step (rewards are non-zero only on
+ *       the terminal step, so this is the per-quad sum).  The output is R[n] in [4]; the caller takes R.mean().
+ * BRL_F_EVAL_FREE_RUN (full statistics only, game_mode "free-run"): team 2 always passes.  Every live row is forwarded by net 0
+ * (team 2's too: brl_model_rows needs no change) and brl_eval_act_log reads no team-2 logits, so the results equal the host
+ * loop's at the cost of forwarding team 2's rows; net 1 is not read.
+ * buffers: [0] in u64 keys[n]  [1] in deal_table  [2] in pool u8[2, brl_mlp_pool_stride()]
+ *          [3] scratch (brl_evaluate_match_scratch_bytes(n, mode))  [4] out f32 cum_return[n] (simple: R[n])
+ *          [5] out f32 acc[n, BRL_EVAL_ACC_COLS] (full statistics; simple: not read)
+ *          [6] inout f64 sums[239] (+= brl_eval_summary; simple: not read)  [7] out i32 status[1] (BRL_MATCH_*)
+ *          [8..13] out final Table_info A, [14..19] B, as brl_duplicate_match [9..20] (duplicate mode: all twelve or none)
+ *          [20] out final state  [21] out bf16 obs[n,480]  [22] out u8 mask[n,38]  [23] out f32 rewards_sum[n,4]
+ *          [24] out u8 terminated[n]  [25] out i8 current_player[n] (single-table mode: all six or none; the state after the
+ *          loop with rewards = the summed rewards, what evaluate returns, :591)
+ * Buffers a mode does not read may be NULL.  Without [8..19] / [20..25] those live in the scratch.
+ * params: n_envs = n, n_deals, illegal_penalty / illegal_bonus as brl_step, flags BRL_F_EVAL_MATCH(mode) |
+ *         BRL_F_EVAL_FREE_RUN | BRL_F_MLP_BF16 | BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED (BRL_F_SAMPLE is an error).
+ * The graph cache and brl_duplicate_match_graph_builds() are shared with brl_duplicate_match. */
+#define BRL_EVAL_MATCH_DUPLICATE 1
+#define BRL_EVAL_MATCH_SINGLE 2
+#define BRL_EVAL_MATCH_SIMPLE 3
+#define BRL_F_EVAL_MATCH(mode) ((mode) << 27)
+#define BRL_EVAL_MATCH_MODE(flags) (((flags) >> 27) & 3)
+#define BRL_F_EVAL_FREE_RUN 0x0008
+int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode);
+int32_t brl_evaluate_match(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -519,6 +561,7 @@ void brl_model_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_t
 void brl_policy_act_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_match_stats_ranges_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_duplicate_match_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_evaluate_match_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_loss_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_clip_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_adam_apply_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
