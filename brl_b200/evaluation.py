@@ -286,9 +286,9 @@ class _MatchBuffers:
     """Fixed-address inputs and outputs of brl_duplicate_match for one shape (n envs, M nets, P ranges; P = 0: one range
     over the batch), so that repeated calls relaunch the op's cached graph instead of capturing a new one."""
 
-    def __init__(self, n: int, M: int, P: int, dev, with_models: bool, with_tables: bool):
+    def __init__(self, n: int, M: int, P: int, dev, with_models: bool, with_tables: bool, pool=None):
         self.keys = torch.empty(n, dtype=torch.int64, device=dev)
-        self.pool = torch.zeros((M, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
+        self.pool = pool if pool is not None else torch.zeros((M, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
         self.env_models = torch.empty((n, 2), dtype=torch.int32, device=dev) if with_models else None
         self.offsets = torch.empty(P + 1, dtype=torch.int64, device=dev) if P else None
         self.scratch = torch.empty(ops.duplicate_match_scratch_bytes(n, M), dtype=torch.uint8, device=dev)
@@ -296,6 +296,15 @@ class _MatchBuffers:
         self.sums = torch.zeros((P, 8) if P else (8,), dtype=torch.float64, device=dev)
         self.status = torch.zeros(1, dtype=torch.int32, device=dev)
         self.tables = (ops.TableInfoBuffers(n, dev), ops.TableInfoBuffers(n, dev)) if with_tables else (None, None)
+
+    def prefix(self, n: int, P: int) -> "_MatchBuffers":
+        """the first n envs and P ranges of these buffers (with env models and ranges, without Table_infos): a smaller shape at
+        the same addresses, whose scratch is large enough because the op's scratch size grows with n"""
+        v = _MatchBuffers.__new__(_MatchBuffers)
+        v.keys, v.env_models, v.cum_return = self.keys[:n], self.env_models[:n], self.cum_return[:n]
+        v.offsets, v.sums = self.offsets[:P + 1], self.sums[:P]
+        v.pool, v.scratch, v.status, v.tables = self.pool, self.scratch, self.status, self.tables
+        return v
 
     def play(self, eval_env, single_bf16: bool, tune: int):
         self.sums.zero_()
@@ -342,60 +351,161 @@ def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_en
     return duplicate_evaluate
 
 
+def pair_chunk_layout(num_pairs: int, n: int, pairs_per_chunk: int, rank: int, world: int):
+    """How the device pair matches lay out `num_pairs` matches of `n` boards each: chunks of `pairs_per_chunk` matches, each
+    chunk's P * n envs sharded over the ranks by global env index g (match g // n, board g % n).  Yields per chunk
+    (c0, P, lo, hi, p_lo, p_hi, bounds): the chunk's first pair, its pair count, this rank's global env range [lo, hi), the
+    matches [p_lo, p_hi) of the chunk that range touches and their local env ranges bounds[p - p_lo] .. bounds[p - p_lo + 1]."""
+    import numpy as np
+    for c0 in range(0, num_pairs, pairs_per_chunk):
+        P = min(pairs_per_chunk, num_pairs - c0)
+        lo, hi = bdist.shard_range(P * n, rank, world)
+        p_lo, p_hi = lo // n, (hi + n - 1) // n
+        bounds = np.clip(np.arange(p_lo, p_hi + 1, dtype=np.int64) * n - lo, 0, hi - lo)
+        yield c0, P, lo, hi, p_lo, p_hi, bounds
+
+
+def _pool_match_shape(max_pairs: int, n: int, pairs_per_chunk: int, world: int):
+    """(envs, ranges) of the largest chunk shard any rank plays for at most `max_pairs` matches of `n` boards"""
+    P = min(max_pairs, pairs_per_chunk)
+    return -(-P * n // world), P
+
+
+def pair_match_bytes(n_envs: int, M: int, P: int) -> int:
+    """device bytes of one set of the pair matches' buffers for n_envs envs, M nets and P ranges (the pool not counted)"""
+    return ops.duplicate_match_scratch_bytes(n_envs, M) + n_envs * (8 + 8 + 4) + 8 * (P + 1) + 64 * P + 4
+
+
+def pfsp_probe_bytes(capacity: int, num_eval_envs: int, max_envs: int = 1 << 20, world: int = 1) -> int:
+    """device bytes make_device_pfsp_probe holds on each of `world` ranks for a zoo of `capacity` models (its pool not
+    counted): one buffer set for the largest chunk over M = 1 + capacity nets"""
+    if capacity == 0:
+        return 0
+    n_envs, P = _pool_match_shape(capacity, num_eval_envs, max(1, (max_envs * world) // num_eval_envs), world)
+    return pair_match_bytes(n_envs, 1 + capacity, P)
+
+
+def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_envs: int, tune: int):
+    """The engine of the device league and the PFSP probe: `matches(pairs, rng_key, params_list=None, pool=None,
+    cum_returns=None)` plays every (i, j) of `pairs` -- net i of the pool on players 0/1, net j on 2/3 -- as the duplicate match
+    `make_simple_duplicate_evaluate(..., num_eval_envs)(net_i, net_j, rng_key)` plays, on the same boards in every match, and
+    returns their (imp, se, win_rate) in `pairs` order.  The nets are `params_list` (packed into a pool of the matches' own)
+    or the caller's packed `pool` (u8[M, brl_mlp_pool_stride()], used in place).  At most `max_envs` envs per rank make one
+    chunk and one brl_duplicate_match call; a chunk's envs are sharded by global index over the ranks (pair_chunk_layout),
+    with one all-reduce of f64[P, 8] and one host read per chunk, so the result does not depend on the rank count.
+    Buffers stay at fixed addresses, so repeated calls relaunch the op's cached graphs: with `params_list` one set per shape;
+    with a caller's pool ONE set, allocated by `matches.reserve(pool, max_pairs)` for the largest chunk of up to `max_pairs`
+    matches (pair_match_bytes of _pool_match_shape), every chunk playing on a prefix of it -- so a pool whose pair count grows
+    call by call (a filling zoo) holds exactly that memory from the reservation on.  `cum_returns` (a dict, tests) receives
+    each pair's per-env returns of this rank's shard."""
+    import numpy as np
+    rank, world = bdist.rank_world()
+    n, dev = num_eval_envs, eval_env.device
+    pairs_per_chunk = max(1, (max_envs * world) // n)
+    buffers = {}
+    held = {}                                                   # the caller pool's set: pool, max_pairs, buffers
+    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+    single_bf16 = forward_pass.precision == "tc-bf16"
+
+    def reserve(pool, max_pairs: int) -> None:
+        if held and held["pool"] is pool and held["max_pairs"] >= max_pairs:
+            return
+        held.clear()                                            # free the previous set before allocating the new one
+        n_envs, P = _pool_match_shape(max_pairs, n, pairs_per_chunk, world)
+        held.update(pool=pool, max_pairs=max_pairs,
+                    buffers=_MatchBuffers(n_envs, pool.shape[0], P, dev, with_models=True, with_tables=False, pool=pool))
+
+    def matches(pairs, rng_key, params_list=None, pool=None, cum_returns=None):
+        M = len(params_list) if pool is None else pool.shape[0]
+        if pool is not None:
+            reserve(pool, len(pairs))
+        _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
+        board_keys = eval_env.make_keys(sub_key, n)
+        pair_arr = np.asarray(pairs, dtype=np.int32).reshape(-1, 2)
+        stats = []
+        for c0, P, lo, hi, p_lo, p_hi, bounds in pair_chunk_layout(len(pairs), n, pairs_per_chunk, rank, world):
+            sums = torch.zeros((P, 8), dtype=torch.float64, device=dev)
+            status = 0
+            if hi > lo:
+                g = np.arange(lo, hi)
+                if pool is not None:
+                    b = held["buffers"].prefix(hi - lo, p_hi - p_lo)
+                else:
+                    key = (hi - lo, M, p_hi - p_lo)
+                    if key not in buffers:
+                        buffers[key] = _MatchBuffers(hi - lo, M, p_hi - p_lo, dev, with_models=True, with_tables=False)
+                    b = buffers[key]
+                    for m, params in enumerate(params_list):
+                        forward_pass.pack_into(params, b.pool[m, :blob_bytes])
+                b.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
+                b.env_models.copy_(torch.as_tensor(pair_arr[c0 + g // n], device=dev))
+                b.offsets.copy_(torch.as_tensor(bounds, device=dev))
+                b.play(eval_env, single_bf16, tune)
+                sums[p_lo:p_hi] = b.sums
+                status = b.status
+                if cum_returns is not None:
+                    for p in range(p_lo, p_hi):
+                        cum_returns[pairs[c0 + p]] = b.cum_return[int(bounds[p - p_lo]):int(bounds[p - p_lo + 1])].clone()
+            bdist.allreduce_sums(sums)
+            host = sums.cpu()
+            _check_match_status(int(status))
+            stats.extend(bdist.stats_from_sums(host[p]) for p in range(P))
+        return stats
+
+    matches.reserve = reserve
+    matches.held = held
+    return matches
+
+
 def make_device_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *,
                                          tune: int = 0):
     """make_selfplay_league_evaluate with one brl_duplicate_match call per chunk: the same pairs, chunks, sharding and
     all-reduce, the same per-env returns, statistics and matrices, with each chunk's loop on the device."""
     import itertools
-
-    import numpy as np
-    forward_pass = make_forward_pass(activation=activation, model_type=model_type)
-    rank, world = bdist.rank_world()
-    n, dev = num_eval_envs, eval_env.device
-    pairs_per_chunk = max(1, (max_envs * world) // n)
-    buffers = {}
-    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+    matches = _make_device_pair_matches(eval_env, make_forward_pass(activation=activation, model_type=model_type),
+                                        num_eval_envs, max_envs, tune)
 
     def league(params_list, rng_key, cum_returns=None):
         M = len(params_list)
         pairs = list(itertools.combinations(range(M), 2))
-        _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
-        board_keys = eval_env.make_keys(sub_key, n)
-        stats = {}
-        for c0 in range(0, len(pairs), pairs_per_chunk):
-            chunk = pairs[c0:c0 + pairs_per_chunk]
-            P = len(chunk)
-            lo, hi = bdist.shard_range(P * n, rank, world)
-            sums = torch.zeros((P, 8), dtype=torch.float64, device=dev)
-            status = 0
-            if hi > lo:
-                g = np.arange(lo, hi)
-                pair_arr = np.asarray(chunk, dtype=np.int32)
-                p_lo, p_hi = lo // n, (hi + n - 1) // n                                  # the matches this shard touches
-                bounds = np.clip(np.arange(p_lo, p_hi + 1, dtype=np.int64) * n - lo, 0, hi - lo)  # their local env ranges
-                key = (hi - lo, M, p_hi - p_lo)
-                if key not in buffers:
-                    buffers[key] = _MatchBuffers(hi - lo, M, p_hi - p_lo, dev, with_models=True, with_tables=False)
-                b = buffers[key]
-                for m, params in enumerate(params_list):
-                    forward_pass.pack_into(params, b.pool[m, :blob_bytes])
-                b.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
-                b.env_models.copy_(torch.as_tensor(pair_arr[g // n], device=dev))
-                b.offsets.copy_(torch.as_tensor(bounds, device=dev))
-                b.play(eval_env, forward_pass.precision == "tc-bf16", tune)
-                sums[p_lo:p_hi] = b.sums
-                status = b.status
-                if cum_returns is not None:
-                    for p in range(p_lo, p_hi):
-                        cum_returns[chunk[p]] = b.cum_return[int(bounds[p - p_lo]):int(bounds[p - p_lo + 1])].clone()
-            bdist.allreduce_sums(sums)
-            host = sums.cpu()
-            _check_match_status(int(status))
-            for p, pair in enumerate(chunk):
-                stats[pair] = bdist.stats_from_sums(host[p])
+        stats = dict(zip(pairs, matches(pairs, rng_key, params_list=params_list, cum_returns=cum_returns)))
         return (stats,) + league_matrices(M, {pair: s[0] for pair, s in stats.items()})
 
     return league
+
+
+def make_device_pfsp_probe(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):
+    """The PFSP probe of ppo.py:412-436 -- the learner against every model of a zoo.ModelZoo -- as one brl_duplicate_match
+    call per chunk over the zoo's own pool (M = 1 + capacity nets, nothing copied per call).  The learner's parameters are
+    re-packed into the zoo's slot 0, and block k of `num_eval_envs` envs plays (0, slot(k)) on the same boards for every k.
+    `probe(current_params, zoo, rng_key) -> [(imp, se, win_rate)] * len(zoo)` in logical zoo order; entry k equals
+    `make_simple_duplicate_evaluate(..., num_eval_envs)(current_params, <zoo model k>, rng_key)[0]`.  The probe holds one
+    buffer set sized for the zoo's capacity (pfsp_probe_bytes), allocated by `probe.reserve(zoo)` or at the first call, so a
+    filling zoo allocates nothing more.  `cum_returns` (a dict, tests) receives model k's per-env returns of this rank's
+    shard under key k."""
+    matches = _make_device_pair_matches(eval_env, make_forward_pass(activation=activation, model_type=model_type),
+                                        num_eval_envs, max_envs, tune)
+
+    def reserve(zoo) -> None:
+        """allocate the probe's buffers for the zoo's whole capacity now (pfsp_probe_bytes); a probe call does it otherwise"""
+        if zoo.capacity:
+            matches.reserve(zoo.pool, zoo.capacity)
+
+    def probe(current_params, zoo, rng_key, cum_returns=None):
+        if len(zoo) == 0:
+            return []
+        reserve(zoo)
+        zoo.set_learner(current_params)
+        pairs = [(0, zoo.slot(k)) for k in range(len(zoo))]
+        by_pair = {} if cum_returns is not None else None
+        stats = matches(pairs, rng_key, pool=zoo.pool, cum_returns=by_pair)
+        if cum_returns is not None:
+            cum_returns.update({k: by_pair[pair] for k, pair in enumerate(pairs) if pair in by_pair})
+        return stats
+
+    probe.reserve = reserve
+    probe.buffers = lambda: matches.held.get("buffers")      # the buffer set the probe holds (tests, memory accounting)
+    return probe
 
 
 # ---- full evaluation statistics (src/evaluation.py:207-1115) --------------------------------------

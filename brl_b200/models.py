@@ -72,6 +72,18 @@ def params_to_numpy(params) -> Dict[str, np.ndarray]:
     return flat
 
 
+class PackedParams:
+    """A net given as its packed blob (u8[brl_mlp_packed_bytes()], what `brl_mlp_pack` writes) instead of an fp32 parameter
+    dict -- how a device-resident model zoo (zoo.ModelZoo) hands out an opponent.  Every ForwardPass method that takes
+    `params` takes one: the forwards read the blob as is, and `pack_into` copies it (device to device)."""
+    __slots__ = ("blob",)
+
+    def __init__(self, blob: torch.Tensor):
+        if blob.dtype != torch.uint8 or blob.dim() != 1 or blob.numel() != ops._lib.load().brl_mlp_packed_bytes():
+            raise ValueError("PackedParams holds one packed blob: u8[brl_mlp_packed_bytes()]")
+        self.blob = blob
+
+
 class ForwardPass:
     """`hk.without_apply_rng(hk.transform(forward_fn))` look-alike: `.apply(params, x)`."""
 
@@ -98,6 +110,8 @@ class ForwardPass:
 
     def _packed(self, params):
         """bf16 hi/lo blob of `params`, re-packed when any tensor was replaced or updated in place."""
+        if isinstance(params, PackedParams):
+            return params.blob
         fixed = params.get("_brl_packed_fixed")  # a caller-owned blob at a fixed address (CUDA-graph rollout)
         if fixed is not None:
             return fixed
@@ -144,7 +158,9 @@ class ForwardPass:
                             env_offset=env_offset, single_bf16=self.precision == "tc-bf16")
 
     def pack_into(self, params, blob: torch.Tensor) -> torch.Tensor:
-        """re-pack `params` into the caller's fixed-address blob"""
+        """re-pack `params` into the caller's fixed-address blob (a PackedParams: a device-to-device copy of its blob)"""
+        if isinstance(params, PackedParams):
+            return blob.copy_(params.blob)
         return ops.mlp_pack([params[name]["w"] for name in LAYERS], [params[name]["b"] for name in LAYERS], out=blob)
 
     def _ensure_scratch(self, n, device):

@@ -14,7 +14,7 @@ from __future__ import annotations
 import os
 import pickle
 import time
-from typing import Callable, List, Optional, Sequence
+from typing import Callable, Optional, Sequence
 
 import numpy as np
 import torch
@@ -22,13 +22,15 @@ import torch
 from . import deals as _deals
 from . import random as brandom
 from .env import BridgeBidding
-from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_simple_evaluate, make_evaluate,
-                         make_evaluate_log, make_simple_duplicate_evaluate, make_simple_evaluate)
+from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_pfsp_probe,
+                         make_device_simple_evaluate, make_evaluate, make_evaluate_log, make_simple_duplicate_evaluate,
+                         make_simple_evaluate)
 from .gae import make_calc_gae
-from .models import LAYERS, init_params, load_params, make_forward_pass
+from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
 from .optim import make_optimizer
 from .roll_out import make_roll_out
 from .update import make_update_step
+from .zoo import ModelZoo, device_zoo_fits
 
 
 def default_config() -> dict:
@@ -149,12 +151,27 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
         opp_params = load_params(config["opp_model_path"], dev) if config["opp_model_path"] else eval_opp_params
     else:
         opp_params = params
-    # past models.  ppo.py keeps them on disk (params-XXXXXXXX.pkl under save_model_path) and loads one at a time; here
-    # they are host-memory NumPy dicts (14.7 MB each, never resident in HBM) and only exist when the league can use them
-    zoo: List[dict] = []
+    # past models.  ppo.py keeps them on disk (params-XXXXXXXX.pkl under save_model_path) and loads one at a time; here they
+    # only exist when the league can use them.  With device_eval they are a zoo.ModelZoo packed in HBM (allocated once for
+    # every save the run makes, up to num_model_zoo): the PFSP probe is one league call and an opponent one device copy.  If
+    # that pool does not fit in free device memory at the start, without device_eval, or when the opponent's forward is not
+    # the tensor-core one (which reads a packed opponent), they are host-memory NumPy dicts (14.7 MB each), copied to the
+    # device one at a time.
     use_zoo = bool(config["self_play"]) and float(config["ratio_model_zoo"]) > 0.0
+    zoo_capacity = min(config["num_model_zoo"], max(0, config["num_updates"] - 1) // config["save_model_interval"])
+    zoo = []
+    probe_envs = config["num_prioritized_envs"] if config["prioritized_fictitious"] else 0
+    if use_zoo and config["device_eval"] and isinstance(opp_forward_pass, ForwardPass) and \
+            device_zoo_fits(zoo_capacity, probe_envs, dev):
+        zoo = ModelZoo(zoo_capacity, dev)
+        if probe_envs:
+            pfsp_probe = make_device_pfsp_probe(eval_env, config["actor_activation"], config["actor_model_type"], probe_envs)
+            pfsp_probe.reserve(zoo)                          # all of the zoo's device memory is taken here, once
+    device_zoo = isinstance(zoo, ModelZoo)
 
-    def zoo_model(k: int) -> dict:
+    def zoo_model(k: int):
+        if device_zoo:
+            return zoo.opponent(k)
         return {name: {kk: torch.as_tensor(v, device=dev) for kk, v in zoo[k][name].items()} for name in LAYERS}
     save_dir = os.path.join(config["log_path"], config["exp_name"], config["save_model_path"])
     if config["save_model"]:
@@ -162,7 +179,9 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
     logs = []
     for i in range(config["num_updates"]):
         if i != 0 and i % config["save_model_interval"] == 0:                                      # ppo.py:351-362
-            if use_zoo:
+            if device_zoo:
+                zoo.append(runner_state[0])                  # keeps the newest zoo_capacity <= num_model_zoo models
+            elif use_zoo:
                 zoo.append(params_to_host(runner_state[0]))
                 zoo[:] = zoo[-config["num_model_zoo"]:]
             if config["save_model"]:
@@ -181,8 +200,12 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
                 if len(zoo) != 0 and np_rng.binomial(1, config["ratio_model_zoo"]):
                     if config["prioritized_fictitious"]:
                         imp_list = np.zeros(len(zoo))
-                        for k in range(len(zoo)):  # one past model on the device at a time
-                            (imp_list[k], _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], zoo_model(k), eval_rng)
+                        if device_zoo:  # the learner against every zoo model in one league call
+                            imp_list[:] = [imp for imp, _, _ in pfsp_probe(runner_state[0], zoo, eval_rng)]
+                        else:
+                            for k in range(len(zoo)):  # one past model on the device at a time
+                                (imp_list[k], _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], zoo_model(k),
+                                                                                         eval_rng)
                         opp_params = zoo_model(int(np_rng.choice(len(zoo), p=pfsp_probabilities(imp_list, config["prior_t"]))))
                     else:
                         opp_params = zoo_model(int(np_rng.integers(len(zoo))))

@@ -10,7 +10,7 @@ gather) and nothing else.
 
 CUDA graph: every op is enqueue-only, so from 4096 envs on (the fused-forward size) the whole T-step rollout is captured
 ONCE per (shape, opponent) into a CUDA graph and replayed: parameters are re-packed into fixed-address blobs before a
-replay, the env state / last observation are copied into the graph's own buffers (device-to-device memcpy), and the
+replay (an opponent given as models.PackedParams, e.g. from zoo.ModelZoo, is copied device to device), the env state / last observation are copied into the graph's own buffers (device-to-device memcpy), and the
 per-rollout PRNG key is a device word XORed into every captured sampling seed (BRL_F_SEED_SALT).  The returned
 trajectory then aliases the graph's buffers: it is valid until the next call of the same roll_out.
 `BRL_ROLLOUT_GRAPH=0` (or `trace=`) selects the plain launch path.
