@@ -25,7 +25,8 @@ OPS = (
 ) + LAZY_OPS
 HOST_API = ("brl_env_create", "brl_env_destroy", "brl_env_init_host", "brl_env_step_host", "brl_env_rollout_host",
             "brl_env_rollout_host_async", "brl_env_wait", "brl_env_trajectory", "brl_env_rollout_host_compact_async",
-            "brl_env_rollout_host_compact", "brl_result16_decode")
+            "brl_env_rollout_host_compact", "brl_result16_decode", "brl_alloc_compressible", "brl_free_compressible",
+            "brl_compressible_granularity", "brl_round_up_granularity")
 MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_scratch_bytes", "brl_mlp_rows_scratch_bytes",
         "brl_xla_layout", "brl_xla_unreported_failures", "brl_eval_num_sums",
         "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset",
@@ -192,8 +193,36 @@ def load():
     L.brl_result16_decode.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     L.brl_env_trajectory.restype = C.c_int32
     L.brl_env_trajectory.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
+    L.brl_alloc_compressible.restype = C.c_void_p
+    L.brl_alloc_compressible.argtypes = [C.c_size_t, C.c_int32, C.POINTER(C.c_int32)]
+    L.brl_free_compressible.restype = None
+    L.brl_free_compressible.argtypes = [C.c_void_p]
+    L.brl_compressible_granularity.restype = C.c_int64
+    L.brl_compressible_granularity.argtypes = [C.c_int32]
+    L.brl_round_up_granularity.restype = C.c_size_t
+    L.brl_round_up_granularity.argtypes = [C.c_size_t, C.c_size_t]
     _LIB = L
     return L
+
+
+class CompressibleBuffer:
+    """`nbytes` of device memory from brl_alloc_compressible (compressible where the device supports it), freed with the
+    object.  torch sees it as u8[nbytes] through __cuda_array_interface__ and keeps it alive as long as a view of it lives."""
+
+    def __init__(self, nbytes: int, device: int):
+        L = load()
+        self.ptr = None  # __del__ of a failed allocation
+        granted = C.c_int32(0)
+        ptr = L.brl_alloc_compressible(nbytes, device, C.byref(granted))
+        if not ptr:
+            raise BrlError(f"brl_alloc_compressible({nbytes}) failed: {L.brl_last_error().decode()}")
+        self.ptr, self.nbytes, self.granted = ptr, nbytes, bool(granted.value)
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "strides": None,
+                                         "version": 3, "stream": None}
+
+    def __del__(self):
+        if self.ptr and _LIB is not None:
+            _LIB.brl_free_compressible(self.ptr)
 
 
 def call(name: str, stream: int, buffers, params) -> None:

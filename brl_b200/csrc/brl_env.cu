@@ -810,7 +810,10 @@ static void launch_rollout_ws(const EnvArgs& a_in, cudaStream_t s) {
     int epb = epb_of[(a.flags >> 16) & 3];
     if (epb == 0) epb = a.n < 8192 ? 16 : 32;  // measured (scripts/exp_rollout_shapes.py)
     int writers = (a.flags >> 21) & 7;
-    if (writers == 0) writers = epb == 8 ? 1 : (epb == 16 ? 2 : (a.balanced ? 4 : 3));  // measured: scripts/exp_ab.py
+    // measured: scripts/exp_ab.py, and for the balanced grid scripts/exp_compressible.py: into compressible trajectories seven
+    // writers beat four (82.4 against 88.6 us per launch at 8192 envs x 32 steps, B200 at 1000 W); into plain memory seven
+    // would lose (98.5 against 89.0 us), as the extra issue rate there only meets the DRAM write-back that compression shrinks
+    if (writers == 0) writers = epb == 8 ? 1 : (epb == 16 ? 2 : (a.balanced ? 7 : 3));
     if (a.flags & BRL_F_OBS_U8) launch_ws_obs<kObsU8>(a, epb, writers, s);
     else if (a.flags & BRL_F_OBS_BF16) launch_ws_obs<kObsBF16>(a, epb, writers, s);
     else launch_ws_obs<kObsF32>(a, epb, writers, s);

@@ -2,7 +2,11 @@
 // library owns the device-resident packed state, the deal table replica and the
 // output staging; callers pass HOST pointers and the copies are part of the call.
 // This is what a non-JAX host (or bench.py's `e2e` leg) calls.
+#include <cuda.h>
+
+#include <mutex>
 #include <new>
+#include <unordered_map>
 
 #include "common.h"
 
@@ -80,9 +84,165 @@ int32_t copy_out(BrlEnv* env, void* obs, uint8_t* mask, float* rewards, uint8_t*
     if (!ok(cudaStreamSynchronize(s), "stream sync")) return BRL_E_LAUNCH;
     return BRL_OK;
 }
+
+// ---- compressible trajectory memory (CUDA virtual-memory API) ---------------------------------------------------------------
+// The driver's entry points are fetched through the runtime, as encode_fn() does for cuTensorMapEncodeTiled: no -lcuda.
+struct Vmm {
+    decltype(&::cuDeviceGet) device_get;
+    decltype(&::cuDeviceGetAttribute) attribute;
+    decltype(&::cuMemGetAllocationGranularity) granularity;
+    decltype(&::cuMemAddressReserve) reserve;
+    decltype(&::cuMemAddressFree) address_free;
+    decltype(&::cuMemCreate) create;
+    decltype(&::cuMemGetAllocationPropertiesFromHandle) properties;
+    decltype(&::cuMemMap) map;
+    decltype(&::cuMemSetAccess) set_access;
+    decltype(&::cuMemUnmap) unmap;
+    decltype(&::cuMemRelease) release;
+    bool loaded;
+};
+
+template <class F>
+bool entry_point(const char* name, F* fn) {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint(name, &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) p = nullptr;
+    *fn = reinterpret_cast<F>(p);
+    return p != nullptr;
+}
+
+const Vmm& vmm() {
+    static const Vmm v = [] {
+        Vmm t = {};
+        t.loaded = entry_point("cuDeviceGet", &t.device_get) && entry_point("cuDeviceGetAttribute", &t.attribute) &&
+                   entry_point("cuMemGetAllocationGranularity", &t.granularity) &&
+                   entry_point("cuMemAddressReserve", &t.reserve) && entry_point("cuMemAddressFree", &t.address_free) &&
+                   entry_point("cuMemCreate", &t.create) &&
+                   entry_point("cuMemGetAllocationPropertiesFromHandle", &t.properties) && entry_point("cuMemMap", &t.map) &&
+                   entry_point("cuMemSetAccess", &t.set_access) && entry_point("cuMemUnmap", &t.unmap) &&
+                   entry_point("cuMemRelease", &t.release);
+        return t;
+    }();
+    return v;
+}
+
+struct Mapping {
+    size_t bytes;
+    int device;
+};
+std::mutex g_map_mutex;
+std::unordered_map<CUdeviceptr, Mapping> g_mappings;  // live brl_alloc_compressible ranges
+
+bool cu_ok(CUresult r, const char* what) {
+    if (r == CUDA_SUCCESS) return true;
+    brl::fail(BRL_E_LAUNCH, "brl_alloc_compressible: %s failed (CUresult %d)", what, (int)r);
+    return false;
+}
+
+// device property (compressible where the device supports it) and granularity; the caller holds `device` current
+bool vmm_prop(int device, CUmemAllocationProp* prop, size_t* gran) {
+    const Vmm& v = vmm();
+    if (!v.loaded) {
+        brl::fail(BRL_E_LAUNCH, "brl_alloc_compressible: the driver lacks the virtual-memory entry points");
+        return false;
+    }
+    CUdevice dev;
+    int compression = 0;
+    if (!cu_ok(v.device_get(&dev, device), "cuDeviceGet") ||
+        !cu_ok(v.attribute(&compression, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, dev), "cuDeviceGetAttribute"))
+        return false;
+    *prop = {};
+    prop->type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop->location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop->location.id = dev;
+    prop->allocFlags.compressionType = compression ? CU_MEM_ALLOCATION_COMP_GENERIC : CU_MEM_ALLOCATION_COMP_NONE;
+    return cu_ok(v.granularity(gran, prop, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED), "cuMemGetAllocationGranularity");
+}
+
+// runs `fn` with `device` current and restores the caller's device afterwards
+template <class F>
+bool on_device(int device, F fn) {
+    int prev = 0;
+    if (!ok(cudaGetDevice(&prev), "cudaGetDevice") || !ok(cudaSetDevice(device), "cudaSetDevice")) return false;
+    const bool r = fn();
+    cudaSetDevice(prev);
+    return r;
+}
 }  // namespace
 
 extern "C" {
+
+size_t brl_round_up_granularity(size_t bytes, size_t granularity) {
+    if (granularity == 0) return bytes;
+    return (bytes + granularity - 1) / granularity * granularity;
+}
+
+int64_t brl_compressible_granularity(int32_t device) {
+    size_t gran = 0;
+    CUmemAllocationProp prop;
+    if (!on_device(device, [&] { return vmm_prop(device, &prop, &gran); })) return -1;
+    return (int64_t)gran;
+}
+
+void* brl_alloc_compressible(size_t bytes, int32_t device, int32_t* granted) {
+    if (granted) *granted = 0;
+    if (bytes == 0) {
+        brl::fail(BRL_E_OPAQUE, "brl_alloc_compressible: bytes must be > 0");
+        return nullptr;
+    }
+    CUdeviceptr ptr = 0;
+    const bool good = on_device(device, [&] {
+        const Vmm& v = vmm();
+        CUmemAllocationProp prop;
+        size_t gran = 0;
+        if (!vmm_prop(device, &prop, &gran)) return false;
+        const size_t size = brl_round_up_granularity(bytes, gran);
+        if (!cu_ok(v.reserve(&ptr, size, gran, 0, 0), "cuMemAddressReserve")) return false;
+        CUmemGenericAllocationHandle h = 0;
+        if (!cu_ok(v.create(&h, size, &prop, 0), "cuMemCreate")) {
+            v.address_free(ptr, size);
+            return false;
+        }
+        // the driver may hand out a plain allocation for a compressible request: report what was granted
+        CUmemAllocationProp got = {};
+        const bool mapped = cu_ok(v.properties(&got, h), "cuMemGetAllocationPropertiesFromHandle") &&
+                            cu_ok(v.map(ptr, size, 0, h, 0), "cuMemMap");
+        v.release(h);  // the mapping keeps the memory alive until cuMemUnmap
+        CUmemAccessDesc access = {};
+        access.location = prop.location;
+        access.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+        if (!mapped || !cu_ok(v.set_access(ptr, size, &access, 1), "cuMemSetAccess")) {
+            if (mapped) v.unmap(ptr, size);
+            v.address_free(ptr, size);
+            return false;
+        }
+        if (granted) *granted = got.allocFlags.compressionType == CU_MEM_ALLOCATION_COMP_GENERIC ? 1 : 0;
+        std::lock_guard<std::mutex> lock(g_map_mutex);
+        g_mappings[ptr] = Mapping{size, device};
+        return true;
+    });
+    return good ? reinterpret_cast<void*>(ptr) : nullptr;
+}
+
+void brl_free_compressible(void* p) {
+    if (p == nullptr) return;
+    Mapping m;
+    {
+        std::lock_guard<std::mutex> lock(g_map_mutex);
+        auto it = g_mappings.find(reinterpret_cast<CUdeviceptr>(p));
+        if (it == g_mappings.end()) return;
+        m = it->second;
+        g_mappings.erase(it);
+    }
+    // unlike cudaFree, unmapping does not wait for the kernels that still write the range
+    on_device(m.device, [&] {
+        cudaDeviceSynchronize();
+        const Vmm& v = vmm();
+        v.unmap(reinterpret_cast<CUdeviceptr>(p), m.bytes);
+        v.address_free(reinterpret_cast<CUdeviceptr>(p), m.bytes);
+        return true;
+    });
+}
 
 BrlEnv* brl_env_create(int64_t n_envs, int64_t env_offset, const uint8_t* deal_table_host, int32_t n_deals,
                        uint64_t seed, int32_t flags) {
@@ -130,7 +290,8 @@ void brl_env_destroy(BrlEnv* env) {
     if (!env || env->magic != kMagic) return;
     cudaFree(env->d_table); cudaFree(env->d_state); cudaFree(env->d_action); cudaFree(env->d_keys);
     cudaFree(env->d_obs); cudaFree(env->d_mask); cudaFree(env->d_rewards); cudaFree(env->d_term); cudaFree(env->d_cur);
-    cudaFree(env->t_obs); cudaFree(env->t_mask); cudaFree(env->t_rewards); cudaFree(env->t_term); cudaFree(env->t_cur);
+    brl_free_compressible(env->t_obs); brl_free_compressible(env->t_mask);
+    cudaFree(env->t_rewards); cudaFree(env->t_term); cudaFree(env->t_cur);
     cudaFree(env->t_action); cudaFree(env->t_uniforms); cudaFree(env->d_stats);
     for (int c = 0; c < 8; ++c) {
         if (env->ev_in[c]) cudaEventDestroy(env->ev_in[c]);
@@ -184,14 +345,17 @@ int32_t brl_env_step_host(BrlEnv* env, const int32_t* action, void* obs, uint8_t
 
 static bool ensure_trajectory(BrlEnv* env, int32_t k) {
     if (env->traj_k >= k) return true;
-    cudaFree(env->t_obs); cudaFree(env->t_mask); cudaFree(env->t_rewards); cudaFree(env->t_term); cudaFree(env->t_cur);
+    brl_free_compressible(env->t_obs); brl_free_compressible(env->t_mask); cudaFree(env->t_rewards); cudaFree(env->t_term); cudaFree(env->t_cur);
     cudaFree(env->t_action); cudaFree(env->t_uniforms);
     env->t_obs = nullptr; env->t_mask = nullptr; env->t_rewards = nullptr; env->t_term = nullptr; env->t_cur = nullptr;
     env->t_action = nullptr; env->t_uniforms = nullptr;
     env->traj_k = 0;
     const size_t rows = (size_t)k * (size_t)env->n;
-    bool good = ok(cudaMalloc(&env->t_obs, rows * env->obs_row_bytes), "malloc traj obs") &&
-                ok(cudaMalloc(&env->t_mask, rows * BRL_NUM_ACTIONS), "malloc traj mask") &&
+    // observation and mask rows are mostly zero: compressible memory (where the device has it) shrinks their write-back
+    int device = 0;
+    bool good = ok(cudaGetDevice(&device), "cudaGetDevice") &&
+                (env->t_obs = brl_alloc_compressible(rows * env->obs_row_bytes, device, nullptr)) != nullptr &&
+                (env->t_mask = static_cast<uint8_t*>(brl_alloc_compressible(rows * BRL_NUM_ACTIONS, device, nullptr))) != nullptr &&
                 ok(cudaMalloc(&env->t_rewards, rows * 16), "malloc traj rewards") &&
                 ok(cudaMalloc(&env->t_term, rows), "malloc traj terminated") &&
                 ok(cudaMalloc(&env->t_cur, rows), "malloc traj current_player") &&

@@ -59,16 +59,36 @@ def new_state(n: int, device) -> torch.Tensor:
     return torch.empty((STATE_PLANES, n, 4), dtype=torch.int32, device=device)
 
 
+def _trajectory(shape, dtype: torch.dtype, device) -> torch.Tensor:
+    """Uninitialised tensor in compressible device memory (brl_alloc_compressible); freed with its last view."""
+    nbytes = dtype.itemsize
+    for d in shape:
+        nbytes *= d
+    if nbytes == 0:
+        return torch.empty(shape, dtype=dtype, device=device)
+    device = torch.device(device)
+    index = device.index if device.index is not None else torch.cuda.current_device()
+    buf = _lib.CompressibleBuffer(nbytes, index)
+    return torch.as_tensor(buf, device=torch.device("cuda", index)).view(dtype).view(shape)
+
+
 class EnvOutputs:
-    """The Env surface brl consumes (src/roll_out.py:72-100): caller-owned output buffers."""
+    """The Env surface brl consumes (src/roll_out.py:72-100): caller-owned output buffers.
+
+    With rows > 0 the observation and mask trajectories ([rows, n, ...], almost all zero bytes) live in compressible
+    device memory, which shrinks their write-back to DRAM; the per-step outputs (rows = 0) come from torch."""
 
     __slots__ = ("observation", "legal_action_mask", "rewards", "terminated", "current_player")
 
     def __init__(self, n: int, device, obs_dtype=torch.float32, rows: int = 0):
         lead = (rows, n) if rows else (n,)
         odt = torch.uint8 if obs_dtype == torch.bool else obs_dtype
-        self.observation = torch.empty(lead + (OBS_DIM,), dtype=odt, device=device)
-        self.legal_action_mask = torch.empty(lead + (NUM_ACTIONS,), dtype=torch.uint8, device=device)
+        if rows:
+            self.observation = _trajectory(lead + (OBS_DIM,), odt, device)
+            self.legal_action_mask = _trajectory(lead + (NUM_ACTIONS,), torch.uint8, device)
+        else:
+            self.observation = torch.empty(lead + (OBS_DIM,), dtype=odt, device=device)
+            self.legal_action_mask = torch.empty(lead + (NUM_ACTIONS,), dtype=torch.uint8, device=device)
         self.rewards = torch.empty(lead + (4,), dtype=torch.float32, device=device)
         self.terminated = torch.empty(lead, dtype=torch.uint8, device=device)
         self.current_player = torch.empty(lead, dtype=torch.int8, device=device)

@@ -625,6 +625,26 @@ void brl_result16_decode(const int16_t *result, int64_t rows, float *rewards, ui
 /* device pointers of the last rollout's trajectory: obs, mask, rewards, terminated, current_player, action */
 int32_t brl_env_trajectory(BrlEnv *env, void **out_ptrs6);
 
+/* -------------------------------------------------------------------------
+ * Trajectory memory.  Observation and mask rows are almost all zero bytes; on
+ * memory mapped with generic compression the L2 compresses such lines on their
+ * way to DRAM, which shrinks a rollout's write-back.  brl_alloc_compressible
+ * reserves address space, creates a physical allocation (compressible when
+ * CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED says the device has it,
+ * a plain one otherwise), maps it read/write for `device` and returns its
+ * address; NULL on failure (brl_last_error).  The size is rounded up to the
+ * allocation granularity.  *granted (may be NULL) = 1 when the driver granted
+ * compression.  brl_free_compressible synchronises the device (as cudaFree
+ * does) and unmaps; NULL and unknown pointers are ignored.  The host-buffer
+ * layer's obs / mask trajectories come from here.
+ * ------------------------------------------------------------------------- */
+void *brl_alloc_compressible(size_t bytes, int32_t device, int32_t *granted);
+void brl_free_compressible(void *ptr);
+/* granularity brl_alloc_compressible rounds to on `device` (bytes; -1 on error) */
+int64_t brl_compressible_granularity(int32_t device);
+/* bytes rounded up to a multiple of granularity (granularity 0: bytes) */
+size_t brl_round_up_granularity(size_t bytes, size_t granularity);
+
 #ifdef __cplusplus
 }
 #endif
