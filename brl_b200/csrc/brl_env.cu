@@ -415,15 +415,24 @@ __device__ __forceinline__ void emit_obs_row_rot(const uint32_t* R, uint32_t q, 
 
 #ifdef BRL_ROLE_TIMING
 __device__ unsigned long long g_role_cycles[8];
-#define BRL_T0() long long _t0 = clock64()
-#define BRL_ACC(slot) do { long long _t1 = clock64(); if (lane == 0) atomicAdd(&g_role_cycles[slot], (unsigned long long)(_t1 - _t0)); _t0 = _t1; } while (0)
+// slots 0-5 of g_role_cycles for phase 0 alone (0-5) and the last phase alone (8-13); 6 / 7: the env warp's / warp 0's
+// prologue, kernel entry to the end of the first barrier
+__device__ unsigned long long g_role_phase_cycles[16];
+#define BRL_TP() const long long _tp = clock64()
+#define BRL_T0() long long _t0 = clock64(); if (lane == 0 && (is_env_warp || warp == 0)) atomicAdd(&g_role_phase_cycles[is_env_warp ? 6 : 7], (unsigned long long)(_t0 - _tp))
+#define BRL_ACC(slot) do { long long _t1 = clock64(); if (lane == 0) { const unsigned long long _d = (unsigned long long)(_t1 - _t0); \
+    atomicAdd(&g_role_cycles[slot], _d); \
+    if (s == 0) atomicAdd(&g_role_phase_cycles[slot], _d); else if (s == a.k_steps) atomicAdd(&g_role_phase_cycles[8 + (slot)], _d); } \
+    _t0 = _t1; } while (0)
 #else
+#define BRL_TP()
 #define BRL_T0()
 #define BRL_ACC(slot)
 #endif
 
 template <int EPB, int OBS>
 __global__ void __launch_bounds__(256) k_rollout_ws(const EnvArgs a) {
+    BRL_TP();
     __shared__ WsTile<EPB> tiles[2];
     __shared__ uint32_t uniforms[2][kUChunk][32];  // action uniforms, double-buffered chunks of kUChunk steps
     __shared__ uint4 row_slots[2 * EPB * 3];
@@ -446,16 +455,26 @@ __global__ void __launch_bounds__(256) k_rollout_ws(const EnvArgs a) {
     uint64_t mask = 0ull;
     unsigned long long n_term = 0;
     long long rew0 = 0;
+    // Launched with programmatic dependent launch (launch_ws_inst): this grid may start while the previous kernel of the
+    // stream drains.  Until pdl_wait() only shared memory and pure functions of the arguments are touched: the zero mask
+    // pads and, in Philox mode, the uniforms of the first chunk of steps (the writers are idle until the first row).
+    pdl_trigger();  // the next launch's blocks take this launch's places as they retire
+    const int k_pre = a.uniforms ? 0 : (a.k_steps < kUChunk ? a.k_steps : kUChunk);
     if (is_env_warp) {
         if (lane < 2) { tiles[0].M[EPB + lane] = 0ull; tiles[1].M[EPB + lane] = 0ull; }
+    } else {
+        for (int r = warp; r < k_pre; r += n_writers)
+            uniforms[0][r][lane] = action_uniform(a.seed, (uint64_t)(a.env_offset + i), a.step + (uint32_t)r);
+    }
+    pdl_wait();  // the previous kernel has completed and its writes (state, deal table, outputs) are visible
+    if (is_env_warp) {
         if (active) {
             load_env(a.state_in, a.stride, i, e);
             cache.prime(e, rs, lane, a.table, a.n_deals);
             mask = env_legal_mask(e);
         }
-    } else if (warp == 0) {
-        uniforms[0][0][lane] = a.uniforms ? (active ? load_uniform(a, i) : 0u)
-                                          : action_uniform(a.seed, (uint64_t)(a.env_offset + i), a.step);
+    } else if (warp == 0 && a.uniforms) {
+        uniforms[0][0][lane] = active ? load_uniform(a, i) : 0u;
     }
     __syncthreads();
     BRL_T0();
@@ -523,7 +542,7 @@ __global__ void __launch_bounds__(256) k_rollout_ws(const EnvArgs a) {
                     // writes), scripts/exp_e2e_gap.py.  The burst for steps s+1 .. s+32 is issued at s = 0, 32, ...: at s = 0
                     // the writers have nothing to store yet, so it hides under the env warp's first step.
                     if (s % kUChunk == 0) load_uniform_burst(a, uniforms, s, i, active, warp, n_writers, lane);
-                } else if (warp == 0) {
+                } else if (warp == 0 && s + 1 >= kUChunk) {  // the first chunk was drawn before pdl_wait()
                     uniforms[((s + 1) / kUChunk) & 1][(s + 1) % kUChunk][lane] =
                         action_uniform(a.seed, (uint64_t)(a.env_offset + i), a.step + (uint32_t)(s + 1));
                 }
@@ -787,7 +806,9 @@ template <int EPB, int OBS>
 static void launch_ws_inst(const EnvArgs& a, int writers, cudaStream_t s) {
     unsigned grid = (unsigned)((a.n + EPB - 1) / EPB);
     if (a.balanced) grid = ((grid + 147u) / 148u) * 148u;  // 148 SMs: same number of blocks on every SM
-    k_rollout_ws<EPB, OBS><<<grid, 32 * (1 + writers), 0, s>>>(a);
+    // every launch waits (pdl_wait) for the complete previous kernel of the stream, so an event or kernel after a
+    // chain of rollouts still sees all of them finished
+    launch_pdl(k_rollout_ws<EPB, OBS>, dim3(grid), dim3(32 * (1 + writers)), 0, s, a);
 }
 template <int OBS>
 static void launch_ws_obs(const EnvArgs& a, int epb, int writers, cudaStream_t s) {
@@ -1097,6 +1118,12 @@ int32_t brl_state_fields(brl_stream_t stream, void** b, const void* opaque, size
 int32_t brl_debug_role_cycles(unsigned long long* out8, int reset) {
     cudaMemcpyFromSymbol(out8, g_role_cycles, sizeof(g_role_cycles));
     if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_role_cycles, z, sizeof(z)); }
+    return 0;
+}
+// the same split by phase: {phase 0: slots 0-5, prologue: 6-7, last phase: 8-13} (g_role_phase_cycles)
+int32_t brl_debug_role_phase_cycles(unsigned long long* out16, int reset) {
+    cudaMemcpyFromSymbol(out16, g_role_phase_cycles, sizeof(g_role_phase_cycles));
+    if (reset) { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(g_role_phase_cycles, z, sizeof(z)); }
     return 0;
 }
 #endif
