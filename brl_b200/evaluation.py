@@ -196,91 +196,6 @@ def league_matrices(num_models: int, pair_imps):
     return win_lose, win_lose_dis, win_lose_clip
 
 
-def make_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20):
-    """workspace/eval_selfplay_league.py's league as batched jobs: every pair (i, j), i < j, in itertools.combinations
-    order plays the match `make_simple_duplicate_evaluate(..., num_eval_envs)(params_list[i], params_list[j], rng_key)`
-    plays (team 1 = i on players 0/1, team 2 = j; env e of every match keyed as local index e).  The matches of a chunk
-    (at most `max_envs` envs per rank) run as ONE env batch: each step, brl_model_rows groups the live rows by acting net
-    (one host read: the padded row count) and brl_policy_act_grouped forwards all nets of the pool at once.  The chunk's
-    envs are sharded by global index over the ranks, with one all-reduce of f64[P, 8] per chunk, so the result does not
-    depend on the rank count.  `league(params_list, rng_key)` returns ({(i, j): (imp, se, win_rate)}, win_lose,
-    win_lose_dis, win_lose_clip); `cum_returns` (a dict, tests) receives each pair's per-env returns of this rank's shard."""
-    import itertools
-
-    import numpy as np
-    forward_pass = make_forward_pass(activation=activation, model_type=model_type)
-    rank, world = bdist.rank_world()
-    n, dev = num_eval_envs, eval_env.device
-    pairs_per_chunk = max(1, (max_envs * world) // n)
-
-    def league(params_list, rng_key, cum_returns=None):
-        M = len(params_list)
-        pairs = list(itertools.combinations(range(M), 2))
-        pool = ops.mlp_pack_pool(params_list, forward_pass.pack_into)
-        single_bf16 = forward_pass.precision == "tc-bf16"
-        _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
-        board_keys = eval_env.make_keys(sub_key, n)
-        stats = {}
-        league.rows_forwarded = 0
-        for c0 in range(0, len(pairs), pairs_per_chunk):
-            chunk = pairs[c0:c0 + pairs_per_chunk]
-            P = len(chunk)
-            lo, hi = bdist.shard_range(P * n, rank, world)
-            sums = torch.zeros((P, 8), dtype=torch.float64, device=dev)
-            if hi > lo:
-                g = np.arange(lo, hi)
-                match = g // n
-                pair_arr = np.asarray(chunk, dtype=np.int32)
-                env_models = torch.as_tensor(pair_arr[match], device=dev).contiguous()
-                p_lo, p_hi = lo // n, (hi + n - 1) // n                                  # the matches this shard touches
-                bounds = np.clip(np.arange(p_lo, p_hi + 1, dtype=np.int64) * n - lo, 0, hi - lo)  # their local env ranges
-                cum_return = _league_chunk(eval_env, board_keys[torch.as_tensor(g % n, device=dev)], env_models, pool,
-                                           single_bf16, league)
-                ops.match_stats_ranges(cum_return, torch.as_tensor(bounds, device=dev), sums[p_lo:p_hi])
-                if cum_returns is not None:
-                    for p in range(p_lo, p_hi):
-                        cum_returns[chunk[p]] = cum_return[int(bounds[p - p_lo]):int(bounds[p - p_lo + 1])].clone()
-            bdist.allreduce_sums(sums)
-            host = sums.cpu()
-            for p, pair in enumerate(chunk):
-                stats[pair] = bdist.stats_from_sums(host[p])
-        return (stats,) + league_matrices(M, {pair: s[0] for pair, s in stats.items()})
-
-    return league
-
-
-def _league_chunk(eval_env, keys, env_models, pool, single_bf16, counter):
-    """duplicate_evaluate's loop (src/evaluation.py:93-169) over the envs of many matches: per-env cum_return"""
-    step_fn = duplicate_step(eval_env.step)
-    state = _bf16_state(eval_env, keys)
-    table_a_info = Table_info.from_state(state)
-    table_b_info = Table_info.from_state(state)
-    dev, n, M = eval_env.device, keys.shape[0], pool.shape[0]
-    cum_return = torch.zeros(n, dtype=torch.float32, device=dev)
-    action = torch.zeros(n, dtype=torch.int32, device=dev)
-    rows = torch.empty(ops.model_rows_capacity(n, M), dtype=torch.int32, device=dev)
-    block_model = torch.empty(rows.shape[0] // 256, dtype=torch.int32, device=dev)
-    counts = torch.empty(M, dtype=torch.int32, device=dev)
-    offsets = torch.empty(M + 1, dtype=torch.int32, device=dev)
-    scratch = torch.empty(ops.policy_grouped_scratch_bytes(n, M), dtype=torch.uint8, device=dev)
-    host = torch.zeros(1, dtype=torch.int32).pin_memory()
-    while True:
-        ops.model_rows(state.current_player, state._terminated_u8, env_models, rows, counts, offsets, block_model)
-        host.copy_(offsets[M:], non_blocking=True)
-        torch.cuda.current_stream(dev).synchronize()
-        n_rows = int(host[0])
-        if n_rows < 0:
-            raise ops._lib.BrlError(f"brl_model_rows: an acting net id is outside [0, {M})")
-        if n_rows == 0:                                                                # :120-122 ~terminated.all()
-            break
-        ops.policy_act_grouped(state.observation, pool, scratch, state._mask_u8, action, rows[:n_rows], block_model,
-                               single_bf16=single_bf16)
-        counter.rows_forwarded += n_rows
-        state, table_a_info, table_b_info = step_fn(state, action, table_a_info, table_b_info)  # :164
-        cum_return += state.rewards[:, 0]                                              # :167-169
-    return cum_return
-
-
 # ---- the device-loop evaluators: one brl_duplicate_match call per match / league chunk (eval.py:53) -------------------------
 class _MatchBuffers:
     """Fixed-address inputs and outputs of brl_duplicate_match for one shape (n envs, M nets, P ranges; P = 0: one range
@@ -386,7 +301,7 @@ def pfsp_probe_bytes(capacity: int, num_eval_envs: int, max_envs: int = 1 << 20,
 
 
 def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_envs: int, tune: int):
-    """The engine of the device league and the PFSP probe: `matches(pairs, rng_key, params_list=None, pool=None,
+    """The engine of the self-play league and the PFSP probe: `matches(pairs, rng_key, params_list=None, pool=None,
     cum_returns=None)` plays every (i, j) of `pairs` -- net i of the pool on players 0/1, net j on 2/3 -- as the duplicate match
     `make_simple_duplicate_evaluate(..., num_eval_envs)(net_i, net_j, rng_key)` plays, on the same boards in every match, and
     returns their (imp, se, win_rate) in `pairs` order.  The nets are `params_list` (packed into a pool of the matches' own)
@@ -457,10 +372,17 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
     return matches
 
 
-def make_device_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *,
-                                         tune: int = 0):
-    """make_selfplay_league_evaluate with one brl_duplicate_match call per chunk: the same pairs, chunks, sharding and
-    all-reduce, the same per-env returns, statistics and matrices, with each chunk's loop on the device."""
+def make_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *,
+                                  tune: int = 0):
+    """workspace/eval_selfplay_league.py's league as batched jobs: every pair (i, j), i < j, in itertools.combinations
+    order plays the match `make_simple_duplicate_evaluate(..., num_eval_envs)(params_list[i], params_list[j], rng_key)`
+    plays (team 1 = i on players 0/1, team 2 = j; env e of every match keyed as local index e).  The matches of a chunk
+    (at most `max_envs` envs per rank) run as ONE env batch in one brl_duplicate_match call over a pool of all the nets: the
+    loop runs on the device, grouping the live rows by acting net each step for the grouped forward.  The chunk's envs are
+    sharded by global index over the ranks, with one all-reduce of f64[P, 8] per chunk, so the result does not depend on the
+    rank count.  `league(params_list, rng_key)` returns ({(i, j): (imp, se, win_rate)}, win_lose, win_lose_dis,
+    win_lose_clip); `cum_returns` (a dict, tests) receives each pair's per-env returns of this rank's shard.  `tune`:
+    BRL_F_TUNE_MLP_* bits pinning the forward's path."""
     import itertools
     matches = _make_device_pair_matches(eval_env, make_forward_pass(activation=activation, model_type=model_type),
                                         num_eval_envs, max_envs, tune)

@@ -23,8 +23,7 @@ from . import deals as _deals
 from . import random as brandom
 from .env import BridgeBidding
 from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_pfsp_probe,
-                         make_device_simple_evaluate, make_evaluate, make_evaluate_log, make_simple_duplicate_evaluate,
-                         make_simple_evaluate)
+                         make_device_simple_evaluate, make_evaluate_log)
 from .gae import make_calc_gae
 from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
 from .optim import make_optimizer
@@ -47,10 +46,7 @@ def default_config() -> dict:
         num_prioritized_envs=100, gamma=1.0, gae_lambda=0.95, clip_eps=0.2, ent_coef=0.001, vf_coef=0.5,
         value_clipping=True, global_gradient_clipping=True, anneal_lr=False, reward_scaling=False, max_grad_norm=0.5,
         reward_scale=7600.0, actor_illegal_action_mask=True, actor_illegal_action_penalty=False,
-        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0,
-        # not in PPOConfig: run the three evaluations of every iteration (train/score, eval/*, the imp_opp / PFSP probes) as
-        # device loops, one brl_evaluate_match / brl_duplicate_match call each, with the same results
-        device_eval=False)
+        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0)
 
 
 def params_to_host(params) -> dict:
@@ -72,19 +68,15 @@ def pfsp_probabilities(imp_list: np.ndarray, prior_t: float) -> np.ndarray:
 
 def make_evaluators(config: dict, eval_env, eval_opp_params):
     """The three evaluators of every iteration (ppo.py:252-283): (train/score vs eval_opp, the imp_opp / PFSP duplicate probe,
-    the eval/* duplicate statistics) -- the host loops, or with config["device_eval"] their device-loop twins."""
+    the eval/* duplicate statistics), each a device loop of one brl_evaluate_match / brl_duplicate_match call.  They give
+    the results of the host loops make_simple_evaluate / make_simple_duplicate_evaluate / make_evaluate."""
     act, mt = config["actor_activation"], config["actor_model_type"]
     opp_act, opp_mt = config["eval_opp_activation"], config["eval_opp_model_type"]
-    if config["device_eval"]:
-        return (make_device_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"],
-                                            team2_params=eval_opp_params),
-                make_device_duplicate_evaluate(eval_env, act, mt, config["num_prioritized_envs"]),
-                make_device_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"],
-                                     duplicate=True, team2_params=eval_opp_params))
-    return (make_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], team2_params=eval_opp_params),
-            make_simple_duplicate_evaluate(eval_env, act, mt, act, mt, config["num_prioritized_envs"]),
-            make_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"], duplicate=True,
-                          team2_params=eval_opp_params))
+    return (make_device_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"],
+                                        team2_params=eval_opp_params),
+            make_device_duplicate_evaluate(eval_env, act, mt, config["num_prioritized_envs"]),
+            make_device_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"],
+                                 duplicate=True, team2_params=eval_opp_params))
 
 
 def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=None, device="cuda",
@@ -152,17 +144,16 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
     else:
         opp_params = params
     # past models.  ppo.py keeps them on disk (params-XXXXXXXX.pkl under save_model_path) and loads one at a time; here they
-    # only exist when the league can use them.  With device_eval they are a zoo.ModelZoo packed in HBM (allocated once for
-    # every save the run makes, up to num_model_zoo): the PFSP probe is one league call and an opponent one device copy.  If
-    # that pool does not fit in free device memory at the start, without device_eval, or when the opponent's forward is not
-    # the tensor-core one (which reads a packed opponent), they are host-memory NumPy dicts (14.7 MB each), copied to the
-    # device one at a time.
+    # only exist when the league can use them.  They are a zoo.ModelZoo packed in HBM (allocated once for every save the run
+    # makes, up to num_model_zoo): the PFSP probe is one league call and an opponent one device copy.  If that pool does not
+    # fit in free device memory at the start, or when the opponent's forward is not the tensor-core one (which reads a packed
+    # opponent), they are host-memory NumPy dicts (14.7 MB each), copied to the device one at a time and probed one match
+    # each.
     use_zoo = bool(config["self_play"]) and float(config["ratio_model_zoo"]) > 0.0
     zoo_capacity = min(config["num_model_zoo"], max(0, config["num_updates"] - 1) // config["save_model_interval"])
     zoo = []
     probe_envs = config["num_prioritized_envs"] if config["prioritized_fictitious"] else 0
-    if use_zoo and config["device_eval"] and isinstance(opp_forward_pass, ForwardPass) and \
-            device_zoo_fits(zoo_capacity, probe_envs, dev):
+    if use_zoo and isinstance(opp_forward_pass, ForwardPass) and device_zoo_fits(zoo_capacity, probe_envs, dev):
         zoo = ModelZoo(zoo_capacity, dev)
         if probe_envs:
             pfsp_probe = make_device_pfsp_probe(eval_env, config["actor_activation"], config["actor_model_type"], probe_envs)

@@ -3,11 +3,11 @@
     python scripts/duplicate_match_bench.py [--reps 10] [--warmup 2] [--out profiles/r04_duplicate_match_b200.json]
 
 Shapes: the configs[0] match (100 boards), the configs[3] match (65,536 boards) -- make_simple_duplicate_evaluate (host
-loop: one host read of the live-row counts per step) against make_device_duplicate_evaluate (one brl_duplicate_match call) --
-and a league chunk of 10 nets (45 matches x 100 boards in one batch): make_selfplay_league_evaluate against
-make_device_selfplay_league_evaluate.  Each timed call is a whole match, from the keys to the statistics on the host, between
-CUDA events; the two loops alternate call by call after `warmup` calls of each, and every timed pair must give bit-equal
-per-env returns.  The card's name and power limit are read in the same run.
+loop: one host read of the live-row counts per step) against make_device_duplicate_evaluate (one brl_duplicate_match call).
+Each timed call is a whole match, from the keys to the statistics on the host, between CUDA events; the two loops alternate
+call by call after `warmup` calls of each, and every timed pair must give bit-equal per-env returns.  The card's name and
+power limit are read in the same run.  The self-play league's former host loop was timed against its device loop here too:
+profiles/r04_duplicate_match_b200.json (10 nets) and profiles/r09_league_host_vs_device_b200.json (10, 21 and 101 nets).
 """
 import argparse
 import json
@@ -20,8 +20,7 @@ import torch
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 from brl_b200 import BridgeBidding, random as brandom  # noqa: E402
 from brl_b200.deals import synthetic_deal_table  # noqa: E402
-from brl_b200.evaluation import (make_device_duplicate_evaluate, make_device_selfplay_league_evaluate,  # noqa: E402
-                                 make_selfplay_league_evaluate, make_simple_duplicate_evaluate)
+from brl_b200.evaluation import make_device_duplicate_evaluate, make_simple_duplicate_evaluate  # noqa: E402
 from brl_b200.models import LAYERS, init_params  # noqa: E402
 
 
@@ -80,17 +79,6 @@ def main():
         devm = make_device_duplicate_evaluate(env, "relu", "DeepMind", n)
         rows.append(compare(f"duplicate_match_{n}", lambda: host(nets[0], nets[1], key), lambda: devm(nets[0], nets[1], key),
                             lambda r: [r[3]], args.reps, args.warmup))
-    league_nets = [seeded_params(910 + m, dev) for m in range(10)]
-    host_l = make_selfplay_league_evaluate(env, "relu", "DeepMind", 100)
-    dev_l = make_device_selfplay_league_evaluate(env, "relu", "DeepMind", 100)
-
-    def run(league):
-        got = {}
-        league(league_nets, key, cum_returns=got)
-        return got
-
-    rows.append(compare("league_10_nets_45x100", lambda: run(host_l), lambda: run(dev_l),
-                        lambda r: [r[p] for p in sorted(r)], args.reps, args.warmup))
     result = {"card": card, "reps": args.reps, "warmup": args.warmup,
               "timing": "CUDA events around whole matches (keys to host statistics), loops alternating", "rows": rows}
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)

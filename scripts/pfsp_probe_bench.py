@@ -12,7 +12,7 @@ that ends in a device synchronise.  After one untimed call of each (its time and
 the one-time capture / instantiate cost when K changes) the two probes alternate call by call, and every pair must give
 the same statistics.  The zoo models are seeded nets with a trained net's logit scale (policy head x 128), drawn on the device.
 
-ppo.train leg: ppo.py's shape (8192 envs x 32 steps, minibatch 1024, 10 epochs), device_eval=True, prioritized_fictitious
+ppo.train leg: ppo.py's shape (8192 envs x 32 steps, minibatch 1024, 10 epochs), prioritized_fictitious
 with ratio_model_zoo = 1 and a save every iteration, run for --train-zoo + 1 iterations so that the last iterations draw
 from a zoo of about --train-zoo models; the host zoo run has the device zoo refused up front.  Per-iteration time is the
 host clock between log_fn calls; with the device zoo each probe call inside the run is timed as
@@ -60,7 +60,7 @@ def probe_leg(env, current, host_zoo, zoo, n, reps, key, dev):
     per_model = make_device_duplicate_evaluate(env, "relu", "DeepMind", n)
     probe = make_device_pfsp_probe(env, "relu", "DeepMind", n)
 
-    def old():   # ppo.train's device_eval probe with the host zoo: zoo_model(k) (H2D) + pack + one match per model
+    def old():   # ppo.train's probe with the host zoo: zoo_model(k) (H2D) + pack + one match per model
         return [per_model(current, {name: {kk: torch.as_tensor(v, device=dev) for kk, v in m[name].items()} for name in LAYERS},
                           key)[0] for m in host_zoo]
 
@@ -117,7 +117,7 @@ def train_leg(device_zoo, zoo_size, dev):
 
     config = dict(num_envs=8192, num_steps=32, minibatch_size=1024, total_timesteps=8192 * 32 * (zoo_size + 1),
                   self_play=True, ratio_model_zoo=1.0, prioritized_fictitious=True, num_model_zoo=zoo_size,
-                  save_model_interval=1, save_model=False, device_eval=True)
+                  save_model_interval=1, save_model=False)
     try:
         _, logs = ppo.train(config, brandom.PRNGKey(0), tables=[synthetic_deal_table(100_000, seed=k) for k in range(2)],
                             eval_table=synthetic_deal_table(10_000, seed=9), device=dev, log_fn=log_fn)

@@ -8,6 +8,7 @@ The arguments are the script's config keys as key=value (SelfplayLeagueConfig). 
 models_directory/exp_name with "params" in the name, step % skip_interval == 0 and step <= max_step, sorted; ppo.train's
 params-XXXXXXXX.pkl qualify, its opt_state-*.pkl do not.  Every pair (i, j), i < j, plays one
 make_simple_duplicate_evaluate match over the same num_eval_envs boards (rng PRNGKey(0)), all matches batched on the GPU
+with each chunk of up to max_envs envs per rank played as one device-resident brl_duplicate_match call
 (evaluation.make_selfplay_league_evaluate).
 
 Writes win_lose_{exp_name}.npy (the reference's output) and win_lose_{exp_name}.npz with win_lose, win_lose_dis,

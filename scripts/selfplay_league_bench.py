@@ -3,11 +3,9 @@ pairwise make_simple_duplicate_evaluate loop.
 
     python scripts/selfplay_league_bench.py [--models 21 101] [--pairwise-models 21] [--boards 100] [--out FILE]
 
-Per M: wall time of league(params_list, rng) (CUDA-synchronised host clock, after one warm-up league on the same M),
-then, in a separate instrumented run, CUDA-event time of every brl_policy_act_grouped call (gather + forward), the padded
-and live forward rows, useful TFLOP/s = live rows x 7,354,368 FLOP / grouped-forward time, and the pool's bytes.  For
---pairwise-models the pairwise loop is timed too and its matrices must equal the league's.  The card's name and power
-limit are read in the same process.  Writes one JSON object (stdout and --out).
+Per M: wall time of league(params_list, rng) (CUDA-synchronised host clock, after one warm-up league on the same M) and
+the pool's bytes.  For --pairwise-models the pairwise loop is timed too and its matrices must equal the league's.  The
+card's name and power limit are read in the same process.  Writes one JSON object (stdout and --out).
 """
 import argparse
 import itertools
@@ -24,8 +22,6 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."
 from brl_b200 import BridgeBidding, evaluation, ops, random as brandom  # noqa: E402
 from brl_b200.deals import synthetic_deal_table  # noqa: E402
 from brl_b200.models import init_params, LAYERS  # noqa: E402
-
-FLOP_PER_ROW = 2 * (480 * 1024 + 3 * 1024 * 1024 + 1024 * 39)  # 7,354,368: the five GEMMs of one forward row
 
 
 def seeded(seed, dev):  # tests/helpers.seeded_params: trained-size logits, so decisions are not near-ties
@@ -51,28 +47,6 @@ def timed(fn):
     return time.perf_counter() - t0, out
 
 
-def instrumented(league, nets, key):
-    """league with CUDA events around every grouped forward; returns (forward ms, padded rows, live rows)"""
-    real = ops.policy_act_grouped
-    events, live = [], torch.zeros((), dtype=torch.int64, device="cuda")
-
-    def wrapped(obs, pool, scratch, mask, action, rows, block_model, *a, **k):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        real(obs, pool, scratch, mask, action, rows, block_model, *a, **k)
-        e1.record()
-        events.append((e0, e1))
-        live.add_((rows >= 0).sum())
-
-    evaluation.ops.policy_act_grouped = wrapped
-    try:
-        league(nets, key)
-    finally:
-        evaluation.ops.policy_act_grouped = real
-    torch.cuda.synchronize()
-    return sum(a.elapsed_time(b) for a, b in events), league.rows_forwarded, int(live), len(events)
-
-
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--models", type=int, nargs="+", default=[21, 101])
@@ -90,10 +64,7 @@ def main():
         nets = [seeded(1000 + m, dev) for m in range(M)]
         league(nets, key)                                                  # warm-up: kernels, tensor maps, allocator
         t_league, (stats, wl, dis, clip) = timed(lambda: league(nets, key))
-        fwd_ms, padded, live, steps = instrumented(league, nets, key)
         run = {"models": M, "matches": len(stats), "boards": len(stats) * a.boards, "league_s": t_league,
-               "loop_iterations": steps, "forward_rows_padded": padded, "forward_rows_live": live,
-               "grouped_forward_ms": fwd_ms, "useful_tflops": live * FLOP_PER_ROW / (fwd_ms * 1e-3) / 1e12,
                "pool_bytes": M * ops.mlp_pool_stride()}
         if M in a.pairwise_models:
             match = evaluation.make_simple_duplicate_evaluate(env, "relu", "DeepMind", "relu", "DeepMind", a.boards)

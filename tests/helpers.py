@@ -39,6 +39,17 @@ def seeded_params(seed, device):
     return p
 
 
+def host_evaluators(config, eval_env, eval_opp_params):
+    """ppo.make_evaluators with the host loops the device evaluators are checked against, built from the same arguments"""
+    from brl_b200.evaluation import make_evaluate, make_simple_duplicate_evaluate, make_simple_evaluate
+    act, mt = config["actor_activation"], config["actor_model_type"]
+    opp_act, opp_mt = config["eval_opp_activation"], config["eval_opp_model_type"]
+    return (make_simple_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], team2_params=eval_opp_params),
+            make_simple_duplicate_evaluate(eval_env, act, mt, act, mt, config["num_prioritized_envs"]),
+            make_evaluate(eval_env, act, mt, opp_act, opp_mt, None, config["num_eval_envs"], config["game_mode"], duplicate=True,
+                          team2_params=eval_opp_params))
+
+
 def weight_path(name):
     """bundled model pickle (bridge_models/ of the reference, 15 MB each): not in the repository; copy it to
     tests/golden/_weights/ (git-ignored) to run the checks that use it"""

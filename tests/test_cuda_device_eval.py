@@ -1,6 +1,6 @@
 """GPU: brl_evaluate_match, make_evaluate / make_simple_evaluate as one device-resident call -- equal to their host loops per
-env and in every statistic, the golden seeded match, the graph cache, capture in a CUDA graph, ppo.train with device_eval and
-the XLA symbol."""
+env and in every statistic, the golden seeded match, the graph cache, capture in a CUDA graph, ppo.train with the device
+evaluators against the same run with the host loops, and the XLA symbol."""
 import numpy as np
 import pytest
 import torch
@@ -222,20 +222,22 @@ def test_xla_symbol_equals_the_direct_call():
     _same(out, ref)
 
 
-def test_ppo_train_with_device_eval_equals_the_host_evaluators():
+def test_ppo_train_with_the_device_evaluators_equals_the_host_evaluators(monkeypatch):
     from brl_b200 import ppo, random as brandom
     from brl_b200.deals import synthetic_deal_table
     from brl_b200.models import params_to_numpy
     config = dict(num_envs=256, num_steps=4, minibatch_size=256, update_epochs=1, total_timesteps=256 * 4 * 3,
                   num_eval_envs=512, num_prioritized_envs=100, num_eval_step=1, self_play=True, ratio_model_zoo=1.0,
                   prioritized_fictitious=True, lr=1e-4, save_model=False)
-    runs = {}
-    for device_eval in (False, True):
-        runs[device_eval] = ppo.train(dict(config, device_eval=device_eval), brandom.PRNGKey(0),
-                                      tables=[synthetic_deal_table(300, seed=k) for k in range(2)],
-                                      eval_table=synthetic_deal_table(400, seed=9), device=DEV,
-                                      eval_opp_params=H.seeded_params(950, DEV))
-    (host_runner, host_logs), (dev_runner, dev_logs) = runs[False], runs[True]
+
+    def run():
+        return ppo.train(config, brandom.PRNGKey(0), tables=[synthetic_deal_table(300, seed=k) for k in range(2)],
+                         eval_table=synthetic_deal_table(400, seed=9), device=DEV, eval_opp_params=H.seeded_params(950, DEV))
+    with monkeypatch.context() as m:   # the host loops, with the host-list zoo and its one match per model
+        m.setattr(ppo, "make_evaluators", H.host_evaluators)
+        m.setattr(ppo, "device_zoo_fits", lambda *a, **kw: False)
+        host_runner, host_logs = run()
+    dev_runner, dev_logs = run()
     assert len(host_logs) == len(dev_logs) == 3
     for h, d in zip(host_logs, dev_logs):
         keys = [k for k in h if k.startswith(("train/score", "train/imp_opp", "eval/"))]

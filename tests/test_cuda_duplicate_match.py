@@ -1,6 +1,6 @@
-"""GPU: brl_duplicate_match, a whole duplicate match as one device-resident call -- bit-equal to the host loops of
-make_selfplay_league_evaluate and make_simple_duplicate_evaluate, the golden seeded match, capture in a CUDA graph, the graph
-cache, the XLA symbol, the bad-net status and the empty batch."""
+"""GPU: brl_duplicate_match, a whole duplicate match as one device-resident call -- bit-equal to the host loop of
+make_simple_duplicate_evaluate, the golden seeded match, capture in a CUDA graph, the graph cache, the XLA symbol, the bad-net
+status and the empty batch.  The self-play league on this op is checked against pairwise host matches in test_cuda_league."""
 import ctypes as C
 
 import numpy as np
@@ -19,41 +19,6 @@ def _env(rows=5000, seed=4):
     from brl_b200 import BridgeBidding
     from brl_b200.deals import synthetic_deal_table
     return BridgeBidding(table=synthetic_deal_table(rows, seed=seed), device=DEV)
-
-
-LEAGUES = [  # (M, boards per match, max_envs, single_bf16): padded live totals above 4096 at the start and below it later
-    (2, 5000, 1 << 20, False),
-    (3, 1000, 3000, False),
-    (3, 1000, 3000, True),
-    (17, 100, 3000, False),
-    (17, 100, 3000, True),
-]
-
-
-@pytest.mark.parametrize("case", range(len(LEAGUES)))
-def test_device_league_equals_the_host_league_loop(case):
-    from brl_b200 import random as brandom
-    from brl_b200.evaluation import make_device_selfplay_league_evaluate, make_selfplay_league_evaluate
-    M, n, max_envs, single_bf16 = LEAGUES[case]
-    env = _env()
-    precision = "tc-bf16" if single_bf16 else "tc"
-    nets = [H.seeded_params(500 + m, DEV) for m in range(M)]
-    key = brandom.PRNGKey(11 + case)
-    host, dev = {}, {}
-    import brl_b200.evaluation as ev
-    orig = ev.make_forward_pass
-    ev.make_forward_pass = lambda **kw: orig(precision=precision, **kw)
-    try:
-        want = make_selfplay_league_evaluate(env, "relu", "DeepMind", n, max_envs=max_envs)(nets, key, cum_returns=host)
-        got = make_device_selfplay_league_evaluate(env, "relu", "DeepMind", n, max_envs=max_envs)(nets, key, cum_returns=dev)
-    finally:
-        ev.make_forward_pass = orig
-    assert list(got[0]) == list(want[0])
-    for pair in want[0]:
-        assert torch.equal(dev[pair], host[pair]), pair
-        assert got[0][pair] == want[0][pair], pair      # integer IMP sums: the statistics are the same numbers
-    for a, b in zip(got[1:], want[1:]):
-        np.testing.assert_array_equal(a, b)
 
 
 def _pin_host_path(monkeypatch, tune):

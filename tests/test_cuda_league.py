@@ -1,6 +1,7 @@
 """GPU: the self-play league (workspace/eval_selfplay_league.py) -- brl_model_rows, the grouped forward over a pool of nets
 (brl_policy_act_grouped) against the one-net listed forward, the batched tournament against pairwise
-make_simple_duplicate_evaluate matches, the golden seeded match, and the XLA symbols of the new ops."""
+make_simple_duplicate_evaluate matches (both precisions, one chunk and several), the golden seeded match, and the XLA symbols of
+the new ops."""
 import ctypes as C
 import itertools
 
@@ -132,16 +133,13 @@ def _script_matrices(M, imps):
     return win_lose, win_lose_dis, win_lose_clip
 
 
-@pytest.mark.parametrize("num_eval_envs", [100, 1000])
-def test_tournament_equals_pairwise_matches(num_eval_envs):
-    from brl_b200 import BridgeBidding, random as brandom
+def _assert_league_equals_pairwise_matches(nets, num_eval_envs, max_envs, key):
+    from brl_b200 import BridgeBidding
     from brl_b200.deals import synthetic_deal_table
     from brl_b200.evaluation import make_selfplay_league_evaluate, make_simple_duplicate_evaluate
     env = BridgeBidding(table=synthetic_deal_table(5000, seed=4), device=DEV)
-    M = 5
-    nets = [H.seeded_params(200 + m, DEV) for m in range(M)]
-    key = brandom.PRNGKey(7)
-    league = make_selfplay_league_evaluate(env, "relu", "DeepMind", num_eval_envs, max_envs=3 * num_eval_envs)  # 4 chunks
+    M = len(nets)
+    league = make_selfplay_league_evaluate(env, "relu", "DeepMind", num_eval_envs, max_envs=max_envs)
     got = {}
     stats, wl, dis, clip = league(nets, key, cum_returns=got)
     match = make_simple_duplicate_evaluate(env, "relu", "DeepMind", "relu", "DeepMind", num_eval_envs)
@@ -150,10 +148,38 @@ def test_tournament_equals_pairwise_matches(num_eval_envs):
     for (i, j), s in stats.items():
         (mean, se, win), _, _, cum = match(nets[i], nets[j], key)
         assert torch.equal(got[(i, j)], cum), (i, j)
-        np.testing.assert_allclose(s, (mean, se, win), rtol=1e-12, atol=0)
+        assert s == (mean, se, win), (i, j)     # integer IMP sums: the statistics are the same numbers
         imps[(i, j)] = mean
     for a, b in zip((wl, dis, clip), _script_matrices(M, imps)):
         np.testing.assert_array_equal(a, b)
+
+
+@pytest.mark.parametrize("num_eval_envs", [100, 1000])
+def test_tournament_equals_pairwise_matches(num_eval_envs):
+    from brl_b200 import random as brandom
+    nets = [H.seeded_params(200 + m, DEV) for m in range(5)]
+    _assert_league_equals_pairwise_matches(nets, num_eval_envs, 3 * num_eval_envs, brandom.PRNGKey(7))  # 4 chunks
+
+
+LEAGUES = [  # (M, boards per match, max_envs, single_bf16): padded live totals above 4096 at the start and below it later
+    (2, 5000, 1 << 20, False),
+    (3, 1000, 3000, False),
+    (3, 1000, 3000, True),
+    (17, 100, 3000, False),
+    (17, 100, 3000, True),
+]
+
+
+@pytest.mark.parametrize("case", range(len(LEAGUES)))
+def test_tournament_equals_pairwise_matches_at_both_precisions(case, monkeypatch):
+    """both the league and the pairwise matches run the precision of the case"""
+    from brl_b200 import random as brandom
+    import brl_b200.evaluation as ev
+    M, n, max_envs, single_bf16 = LEAGUES[case]
+    orig = ev.make_forward_pass
+    monkeypatch.setattr(ev, "make_forward_pass", lambda **kw: orig(precision="tc-bf16" if single_bf16 else "tc", **kw))
+    nets = [H.seeded_params(500 + m, DEV) for m in range(M)]
+    _assert_league_equals_pairwise_matches(nets, n, max_envs, brandom.PRNGKey(11 + case))
 
 
 def test_tournament_reproduces_the_golden_seeded_match():

@@ -115,13 +115,12 @@ def test_rollout_with_a_packed_opponent_equals_fp32_params(graph, monkeypatch):
         assert torch.equal(out[0][1], other[1]) and out[0][2:] == other[2:]
 
 
-def _train(device_eval, prioritized, zoo_size):
+def _train(prioritized, zoo_size):
     from brl_b200 import ppo, random as brandom
     from brl_b200.deals import synthetic_deal_table
     config = dict(num_envs=4096, num_steps=2, minibatch_size=2048, update_epochs=1, total_timesteps=4096 * 2 * 6,
                   num_eval_envs=512, num_prioritized_envs=100, num_eval_step=3, self_play=True, ratio_model_zoo=1.0,
-                  num_model_zoo=zoo_size, save_model_interval=1, prioritized_fictitious=prioritized, lr=1e-4, save_model=False,
-                  device_eval=device_eval)
+                  num_model_zoo=zoo_size, save_model_interval=1, prioritized_fictitious=prioritized, lr=1e-4, save_model=False)
     return ppo.train(config, brandom.PRNGKey(2), tables=[synthetic_deal_table(300, seed=k) for k in range(2)],
                      eval_table=synthetic_deal_table(400, seed=9), device=DEV, eval_opp_params=_net(850))
 
@@ -141,10 +140,11 @@ def _assert_same_run(a, b):
 
 @pytest.mark.parametrize("zoo_size", [1, 2])
 @pytest.mark.parametrize("prioritized", [True, False])
-def test_ppo_train_with_the_device_zoo_equals_the_host_zoo(prioritized, zoo_size, monkeypatch):
+def test_ppo_train_with_the_device_zoo_equals_the_host_list_zoo(prioritized, zoo_size, monkeypatch):
     """six iterations, a save every iteration and a one- or two-model zoo, so the ring wraps; the runs contain an append that
-    reuses the slot of the opponent chosen in the iteration before, which that iteration's imp_opp probe still plays.  Then
-    the same run with the device zoo refused by the memory budget."""
+    reuses the slot of the opponent chosen in the iteration before, which that iteration's imp_opp probe still plays.  The
+    reference run plays the host loops with the host-list zoo.  Then the same run with the device zoo refused by the memory
+    budget."""
     import brl_b200.ppo as ppo
     from brl_b200.zoo import ModelZoo
     made, events = [], []
@@ -175,9 +175,12 @@ def test_ppo_train_with_the_device_zoo_equals_the_host_zoo(prioritized, zoo_size
         counted.reserve = probe.reserve
         return counted
     monkeypatch.setattr(ppo, "make_device_pfsp_probe", counting_probe)
-    host = _train(False, prioritized, zoo_size)
+    with monkeypatch.context() as m:   # the host loops, with the host-list zoo and its one match per model
+        m.setattr(ppo, "make_evaluators", H.host_evaluators)
+        m.setattr(ppo, "device_zoo_fits", lambda *a, **kw: False)
+        host = _train(prioritized, zoo_size)
     assert not made
-    device = _train(True, prioritized, zoo_size)
+    device = _train(prioritized, zoo_size)
     assert len(made) == 1 and made[0].capacity == zoo_size and len(made[0]) == zoo_size
     assert len(probes) == (5 if prioritized else 0)                    # one call per PFSP draw (iterations 1..5)
     assert [e for e in events if e[0] == "opponent"]
@@ -187,6 +190,6 @@ def test_ppo_train_with_the_device_zoo_equals_the_host_zoo(prioritized, zoo_size
     _assert_same_run(host, device)
     free, total = torch.cuda.mem_get_info(DEV)
     monkeypatch.setattr(torch.cuda, "mem_get_info", lambda device=None: (1 << 30, total))
-    fallback = _train(True, prioritized, zoo_size)
+    fallback = _train(prioritized, zoo_size)
     assert len(made) == 1 and len(probes) == (5 if prioritized else 0)
     _assert_same_run(host, fallback)

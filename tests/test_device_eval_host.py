@@ -1,5 +1,5 @@
 """CPU: the host side of brl_evaluate_match (make_evaluate / make_simple_evaluate as one device-resident call) -- its XLA
-layout, lazy binding, argument validation, scratch-size query, and ppo.train's evaluator selection."""
+layout, lazy binding, argument validation, scratch-size query, and the evaluators ppo.train builds."""
 import ctypes
 import os
 import subprocess
@@ -130,16 +130,13 @@ def test_python_wrapper_checks_shapes_and_scratch_before_touching_the_device():
         ops.evaluate_match(keys, table, pool2, small, cum, status, mode=_lib.EVAL_MATCH_DUPLICATE, acc=acc, sums=sums)
 
 
-def test_device_eval_defaults_to_the_host_evaluators(monkeypatch):
-    """ppo.train's evaluator selection: the host loops unless config["device_eval"], and then the three device twins"""
+def test_ppo_train_builds_the_device_evaluators(monkeypatch):
+    """ppo.train's evaluators: the three device loops, whatever the config"""
     from brl_b200 import ppo
     made = []
-    for name in ("make_simple_evaluate", "make_simple_duplicate_evaluate", "make_evaluate", "make_device_simple_evaluate",
-                 "make_device_duplicate_evaluate", "make_device_evaluate"):
+    for name in ("make_device_simple_evaluate", "make_device_duplicate_evaluate", "make_device_evaluate"):
         monkeypatch.setattr(ppo, name, lambda *a, _name=name, **kw: made.append(_name) or _name)
     cfg = ppo.default_config()
-    assert cfg["device_eval"] is False
-    assert ppo.make_evaluators(cfg, None, None) == ("make_simple_evaluate", "make_simple_duplicate_evaluate", "make_evaluate")
-    cfg["device_eval"] = True
     assert ppo.make_evaluators(cfg, None, None) == ("make_device_simple_evaluate", "make_device_duplicate_evaluate",
                                                     "make_device_evaluate")
+    assert made == ["make_device_simple_evaluate", "make_device_duplicate_evaluate", "make_device_evaluate"]
