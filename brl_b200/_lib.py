@@ -51,7 +51,7 @@ F_RESULT_I16 = 0x1000
 F_UNIFORM_U16 = 0x2000
 F_SEED_SALT = 0x4000
 F_COUNT_DONE = 0x8000
-ABI_VERSION = 2  # include/brl_b200.h BRL_ABI_VERSION; load() refuses a library built from other headers
+ABI_VERSION = 3  # include/brl_b200.h BRL_ABI_VERSION; load() refuses a library built from other headers
 EVAL_ACC_COLS = 76
 MATCH_MAX_STEPS = 638  # brl_duplicate_match's bound on forwards (BRL_MATCH_MAX_STEPS)
 MATCH_OK, MATCH_BAD_MODEL, MATCH_STEP_BOUND = 0, 1, 2  # its status codes (BRL_MATCH_*)

@@ -33,10 +33,10 @@
 
 namespace brl {
 
-int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
-                                  const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
-                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits);
-int32_t warm_policy_grouped_dev(bool split);
+int32_t launch_policy_grouped(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
+                              const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
+                              const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits);
+int32_t warm_policy_grouped(bool split);
 
 // ---- kernels -----------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_pair_models(int32_t* __restrict__ env_models, int64_t n) {  // every env: net 0 vs net 1
@@ -265,9 +265,9 @@ static int32_t capture_into(const char* who, cudaGraph_t body, cudaStream_t side
 
 static int32_t forward(const MatchPlan& q, cudaStream_t s, int32_t path_flag) {
     const int32_t flags = (q.flags & BRL_F_MLP_BF16) | path_flag;
-    return launch_policy_grouped_dev(s, flags, q.cap, q.M, q.obs, q.pool, q.at<unsigned char>(q.L.forward), static_cast<uint8_t*>(q.mask),
-                                     q.at<int32_t>(q.L.action), q.at<int32_t>(q.L.rows), q.at<int32_t>(q.L.block_model),
-                                     q.offsets() + q.M, q.logits);
+    return launch_policy_grouped(s, flags, q.cap, q.M, q.obs, q.pool, q.at<unsigned char>(q.L.forward), static_cast<uint8_t*>(q.mask),
+                                 q.at<int32_t>(q.L.action), q.at<int32_t>(q.L.rows), q.at<int32_t>(q.L.block_model),
+                                 q.offsets() + q.M, q.logits);
 }
 
 // the env step of one iteration: brl_duplicate_step on both tables (:164, :772-774), or brl_step without auto-reset (:406;
@@ -453,7 +453,7 @@ static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p,
     MatchCache& c = cache();
     std::lock_guard<std::mutex> lock(c.mu);
     cudaStream_t* side = nullptr;
-    if ((rc = warm_policy_grouped_dev(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(q.who, &side))) return rc;
+    if ((rc = warm_policy_grouped(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(q.who, &side))) return rc;
     if (st == cudaStreamCaptureStatusActive) {  // the caller's capture: the nodes go there
         if ((rc = emit_match(q, s, side[1], side[2]))) return rc;
         return check_launch(q.who);

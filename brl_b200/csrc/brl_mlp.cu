@@ -260,24 +260,21 @@ struct LayerArgs {
     int n_tiles_n, n_tiles;      // tiles along N, total tiles of this layer
 };
 // grouped forward (a pool of nets): rows [b * kGroupRows, (b + 1) * kGroupRows) use model block_model[b]; the pool's biases are
-// bias_stride floats apart; the grouped head runs the masked argmax of `act` in its epilogue.  A separate type, so that the
-// ungrouped kernels keep their parameter block (and their code) as it was.
+// bias_stride floats apart; the grouped head runs the masked argmax of `act` in its epilogue.  The row count is read from device
+// memory: the launch and its tensor maps are sized for the grouping's capacity, and the row blocks past the count exit at once.
+// A separate type, so that the ungrouped kernels keep their parameter block (and their code) as it was.
 struct GroupedLayerArgs : LayerArgs {
     const int32_t* block_model;
     int64_t bias_stride;
     ActArgs act;
-};
-// DEVCOUNT (brl_duplicate_match's device loop): the grouped forward's row count is read from device memory; the launch and
-// its tensor maps are sized for the grouping's capacity, and the row blocks past the count exit at once
-struct DevLayerArgs : GroupedLayerArgs {
     const int32_t* n_rows;  // padded row count (brl_model_rows' offsets[M])
 };
-template <bool GROUPED, bool DEVCOUNT = false>
-using LayerArgsT = std::conditional_t<DEVCOUNT, DevLayerArgs, std::conditional_t<GROUPED, GroupedLayerArgs, LayerArgs>>;
+template <bool GROUPED>
+using LayerArgsT = std::conditional_t<GROUPED, GroupedLayerArgs, LayerArgs>;
 __device__ __forceinline__ int layer_rows(const LayerArgs& a) { return a.M; }
-__device__ __forceinline__ int layer_rows(const DevLayerArgs& a) { return *a.n_rows; }
+__device__ __forceinline__ int layer_rows(const GroupedLayerArgs& a) { return *a.n_rows; }
 __device__ __forceinline__ int layer_tiles(const LayerArgs& a) { return a.n_tiles; }
-__device__ __forceinline__ int layer_tiles(const DevLayerArgs& a) { return a.n_tiles_n * ((*a.n_rows + kBM - 1) / kBM); }
+__device__ __forceinline__ int layer_tiles(const GroupedLayerArgs& a) { return a.n_tiles_n * ((*a.n_rows + kBM - 1) / kBM); }
 
 template <int BN, bool SPLIT_A, bool SPLIT_W>
 struct LayerCfg {
@@ -287,11 +284,11 @@ struct LayerCfg {
     static constexpr uint32_t kSmemBytes = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
 __global__ void __launch_bounds__(kMlpThreads, 1)
 k_mlp_layer(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
             const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo,
-            const LayerArgsT<GROUPED, DEVCOUNT> a) {
+            const LayerArgsT<GROUPED> a) {
     // PERSISTENT: one CTA per SM walks tiles blockIdx.x, blockIdx.x + gridDim.x, ... (n-tile fastest, so the
     // CTAs running together share A row-blocks in L2).  The smem stage ring runs straight across tile
     // boundaries and the accumulator is double-buffered in TMEM, so the epilogue of tile j overlaps the
@@ -476,15 +473,13 @@ struct FusedArgs {
     int M, nmb, tiles_per_layer, n_tiles;
     ActArgs act;
 };
-struct GroupedFusedArgs : FusedArgs {  // grouped forward (see GroupedLayerArgs)
+struct GroupedFusedArgs : FusedArgs {  // grouped forward (see GroupedLayerArgs): M, nmb and the tile list follow *n_rows
     const int32_t* block_model;  // model of each kGroupRows-row block (= the CTA-pair tile height)
     int64_t bias_stride;         // floats between two nets' biases in the pool
-};
-struct DevFusedArgs : GroupedFusedArgs {  // DEVCOUNT (see DevLayerArgs): M, nmb and the tile list follow *n_rows
     const int32_t* n_rows;
 };
-template <bool GROUPED, bool DEVCOUNT = false>
-using FusedArgsT = std::conditional_t<DEVCOUNT, DevFusedArgs, std::conditional_t<GROUPED, GroupedFusedArgs, FusedArgs>>;
+template <bool GROUPED>
+using FusedArgsT = std::conditional_t<GROUPED, GroupedFusedArgs, FusedArgs>;
 
 constexpr int kFusedBN = 256, kFusedTilesN = kHidden / kFusedBN;
 // Epilogue warps of the fused forward: TWO per TMEM lane quadrant, each draining half of the tile's 256 columns.  One
@@ -541,22 +536,21 @@ __device__ __forceinline__ const float* fused_bias(const GroupedFusedArgs& a, in
     return a.bias[layer] + (size_t)a.block_model[mb] * a.bias_stride;
 }
 __device__ __forceinline__ bool fused_row_ok(const FusedArgs& a, int row) { return row < a.M; }
-__device__ __forceinline__ bool fused_row_ok(const GroupedFusedArgs& a, int row) { return row < a.M && a.act.row_index[row] >= 0; }
+__device__ __forceinline__ bool fused_row_ok(const GroupedFusedArgs& a, int row) { return row < *a.n_rows && a.act.row_index[row] >= 0; }
 
-// the launch's shape -- rows, 256-row blocks, tiles per hidden layer, tiles -- from the parameters, or (DEVCOUNT) from *n_rows
+// the launch's shape -- rows, 256-row blocks, tiles per hidden layer, tiles -- from the parameters, or (grouped) from *n_rows
 __device__ __forceinline__ int fused_rows(const FusedArgs& a) { return a.M; }
-__device__ __forceinline__ int fused_rows(const DevFusedArgs& a) { return *a.n_rows; }
+__device__ __forceinline__ int fused_rows(const GroupedFusedArgs& a) { return *a.n_rows; }
 __device__ __forceinline__ int fused_nmb(const FusedArgs& a) { return a.nmb; }
-__device__ __forceinline__ int fused_nmb(const DevFusedArgs& a) { return (*a.n_rows + 2 * kBM - 1) / (2 * kBM); }
+__device__ __forceinline__ int fused_nmb(const GroupedFusedArgs& a) { return (*a.n_rows + 2 * kBM - 1) / (2 * kBM); }
 __device__ __forceinline__ int fused_tiles_per_layer(const FusedArgs& a) { return a.tiles_per_layer; }
-__device__ __forceinline__ int fused_tiles_per_layer(const DevFusedArgs& a) { return fused_nmb(a) * kFusedTilesN; }
+__device__ __forceinline__ int fused_tiles_per_layer(const GroupedFusedArgs& a) { return fused_nmb(a) * kFusedTilesN; }
 __device__ __forceinline__ int fused_n_tiles(const FusedArgs& a) { return a.n_tiles; }
-__device__ __forceinline__ int fused_n_tiles(const DevFusedArgs& a) { return fused_nmb(a) * (4 * kFusedTilesN + 1); }
-__device__ __forceinline__ bool fused_row_ok(const DevFusedArgs& a, int row) { return row < *a.n_rows && a.act.row_index[row] >= 0; }
+__device__ __forceinline__ int fused_n_tiles(const GroupedFusedArgs& a) { return fused_nmb(a) * (4 * kFusedTilesN + 1); }
 
-template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
+template <bool SPLIT, bool GROUPED = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kFusedThreads, 1)
-k_mlp_fused(const __grid_constant__ FusedArgsT<GROUPED, DEVCOUNT> a) {
+k_mlp_fused(const __grid_constant__ FusedArgsT<GROUPED> a) {
     using Cfg = FusedCfg<SPLIT>;
     constexpr int S = Cfg::kStages;
     constexpr uint32_t kTmemCols = 2 * kFusedBN;
@@ -735,7 +729,7 @@ struct PoolArgs {
     int64_t stride;
     int n_models;
     ActArgs act;  // the per-layer head's masked argmax (the fused head takes launch_fused's `act`)
-    const int32_t* n_rows;  // DEVCOUNT: the padded row count in device memory (the launch is sized for M = the capacity)
+    const int32_t* n_rows;  // the padded row count in device memory (the launch is sized for M = the capacity)
 };
 
 // weight operand of layer-tile loads: one net's [n_rows, k_in] bf16 matrix, or the pool's {k_in, n_rows, model} stack of them
@@ -749,13 +743,13 @@ static bool make_w_map(CUtensorMap* m, const void* w, uint64_t n_rows, uint64_t 
 
 // the kernel's shared-memory attribute, set once per device (idempotent, a race only repeats the call); also called ahead of a
 // stream capture (brl_duplicate_match) so that no attribute call falls inside one
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
 static int32_t layer_attr() {
     using Cfg = LayerCfg<BN, SPLIT_A, SPLIT_W>;
     static bool attr_set_dev[kMaxDevices] = {};
     bool& attr_set = attr_set_dev[device_slot()];
     if (!attr_set) {
-        if (cudaFuncSetAttribute(k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        if (cudaFuncSetAttribute(k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)Cfg::kSmemBytes) != cudaSuccess)
             return fail(BRL_E_LAUNCH, "brl_mlp_forward: cannot reserve %u bytes of shared memory", Cfg::kSmemBytes);
         attr_set = true;
@@ -763,7 +757,7 @@ static int32_t layer_attr() {
     return BRL_OK;
 }
 
-template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false, bool DEVCOUNT = false>
+template <int BN, bool SPLIT_A, bool SPLIT_W, bool HEAD, bool GROUPED = false>
 static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, int k_in, const void* w_hi, const void* w_lo,
                             int n_valid_rows, const LayerArgs& args, const PoolArgs* pool = nullptr) {
     using Cfg = LayerCfg<BN, SPLIT_A, SPLIT_W>;
@@ -775,16 +769,16 @@ static int32_t launch_layer(cudaStream_t s, const void* a_hi, const void* a_lo, 
     if (ok && SPLIT_A) ok = make_map(&ta_lo, a_lo, (uint64_t)args.M, (uint64_t)k_in, (uint64_t)k_in, kBM);
     if (ok && SPLIT_W) ok = make_w_map<GROUPED>(&tw_lo, w_lo, (uint64_t)n_valid_rows, (uint64_t)k_in, BN, pool);
     if (!ok) return fail(BRL_E_LAUNCH, "brl_mlp_forward: cuTensorMapEncodeTiled failed");
-    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>;
-    if (int32_t rc = layer_attr<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED, DEVCOUNT>()) return rc;
-    LayerArgsT<GROUPED, DEVCOUNT> la{};
+    auto kern = k_mlp_layer<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED>;
+    if (int32_t rc = layer_attr<BN, SPLIT_A, SPLIT_W, HEAD, GROUPED>()) return rc;
+    LayerArgsT<GROUPED> la{};
     static_cast<LayerArgs&>(la) = args;
     if constexpr (GROUPED) {
         la.block_model = pool->block_model;
         la.bias_stride = pool->stride / (int64_t)sizeof(float);
         la.act = pool->act;
+        la.n_rows = pool->n_rows;
     }
-    if constexpr (DEVCOUNT) la.n_rows = pool->n_rows;
     la.n_tiles_n = (n_valid_rows + BN - 1) / BN;
     la.n_tiles = la.n_tiles_n * ((args.M + kBM - 1) / kBM);
     const int n_sm = sm_count();
@@ -798,10 +792,10 @@ static inline size_t fused_ready_bytes(int64_t n_envs) { return (size_t)(4 * 2 *
 
 // co-resident CTA pairs of the fused kernel (the dependency waits need every launched pair to be running), with its shared-memory
 // attribute set on the first call per device; also called ahead of a stream capture (brl_duplicate_match).  0 = failure.
-template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
+template <bool SPLIT, bool GROUPED = false>
 static int fused_pairs() {
     using Cfg = FusedCfg<SPLIT>;
-    auto kern = k_mlp_fused<SPLIT, GROUPED, DEVCOUNT>;
+    auto kern = k_mlp_fused<SPLIT, GROUPED>;
     static int max_pairs_dev[kMaxDevices] = {};
     int& max_pairs = max_pairs_dev[device_slot()];
     if (max_pairs == 0) {
@@ -831,12 +825,12 @@ static int fused_pairs() {
     return max_pairs;
 }
 
-template <bool SPLIT, bool GROUPED = false, bool DEVCOUNT = false>
+template <bool SPLIT, bool GROUPED = false>
 static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char* blob, const MlpLayout& L, __nv_bfloat16* const buf_hi[2],
                             __nv_bfloat16* const buf_lo[2], uint32_t* ready, float* logits, float* value, int M, const ActArgs& act,
                             const PoolArgs* pool = nullptr) {
     using Cfg = FusedCfg<SPLIT>;
-    FusedArgsT<GROUPED, DEVCOUNT> fa{};
+    FusedArgsT<GROUPED> fa{};
     bool ok = true;
     for (int l = 0; l < 5 && ok; ++l) {
         const void* a_hi = l == 0 ? obs : (const void*)buf_hi[(l - 1) & 1];
@@ -866,14 +860,14 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
     if constexpr (GROUPED) {
         fa.block_model = pool->block_model;
         fa.bias_stride = pool->stride / (int64_t)sizeof(float);
+        fa.n_rows = pool->n_rows;
     }
-    if constexpr (DEVCOUNT) fa.n_rows = pool->n_rows;
     fa.M = M;
     fa.nmb = (M + 2 * kBM - 1) / (2 * kBM);
     fa.tiles_per_layer = fa.nmb * kFusedTilesN;
     fa.n_tiles = 4 * fa.tiles_per_layer + fa.nmb;
-    auto kern = k_mlp_fused<SPLIT, GROUPED, DEVCOUNT>;
-    const int max_pairs = fused_pairs<SPLIT, GROUPED, DEVCOUNT>();
+    auto kern = k_mlp_fused<SPLIT, GROUPED>;
+    const int max_pairs = fused_pairs<SPLIT, GROUPED>();
     if (max_pairs == 0) return BRL_E_LAUNCH;
     if (cudaMemsetAsync(ready, 0, fused_ready_bytes(M), s) != cudaSuccess) return check_launch("brl_mlp_forward (memset)");
     const int n_pairs = fa.n_tiles < max_pairs ? fa.n_tiles : max_pairs;
@@ -881,26 +875,19 @@ static int32_t launch_fused(cudaStream_t s, const void* obs, const unsigned char
     return BRL_OK;
 }
 
-// PADDED: index -1 marks a padding row of a grouped batch, gathered as zeros
-template <bool PADDED = false>
 __global__ void __launch_bounds__(256) k_gather_obs_rows(const uint4* __restrict__ src, const int32_t* __restrict__ index,
                                                          uint4* __restrict__ dst, int64_t n, int w) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n * w) return;
     const int64_t r = i / w;
     const int c = (int)(i - r * w);
-    if constexpr (PADDED) {
-        const int32_t e = index[r];
-        dst[i] = e >= 0 ? src[(int64_t)e * w + c] : make_uint4(0u, 0u, 0u, 0u);
-    } else {
-        dst[i] = src[(int64_t)index[r] * w + c];
-    }
+    dst[i] = src[(int64_t)index[r] * w + c];
 }
 
-// the grouped gather of brl_duplicate_match's device loop: launched for the grouping's capacity, it reads the padded row count
-// from device memory and the threads past it exit
-__global__ void __launch_bounds__(256) k_gather_obs_rows_dev(const uint4* __restrict__ src, const int32_t* __restrict__ index,
-                                                             uint4* __restrict__ dst, const int32_t* __restrict__ n_rows, int w) {
+// the grouped gather: launched for the grouping's capacity, it reads the padded row count from device memory and the threads
+// past it exit; index -1 marks a padding row of a group, gathered as zeros
+__global__ void __launch_bounds__(256) k_gather_obs_rows_grouped(const uint4* __restrict__ src, const int32_t* __restrict__ index,
+                                                                 uint4* __restrict__ dst, const int32_t* __restrict__ n_rows, int w) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int64_t)*n_rows * w) return;
     const int64_t r = i / w;
@@ -966,10 +953,11 @@ static bool fused_forward(const BrlParams* p) {
     return (p->flags & BRL_F_TUNE_MLP_FUSED) != 0 || p->n_envs >= kPairMinM;
 }
 
-// forward (+ optional fused categorical) shared by brl_mlp_forward and brl_policy_act.  GROUPED (brl_policy_act_grouped): `blob`
-// is a pool of nets, row block b of the batch runs net pool->block_model[b], and the head epilogue writes action / logits by env
-// (the per-layer head included: no categorical launch).
-template <bool GROUPED = false, bool DEVCOUNT = false>
+// forward (+ optional fused categorical) shared by brl_mlp_forward, brl_policy_act and brl_policy_act_rows.  GROUPED
+// (launch_policy_grouped): `blob` is a pool of nets, row block b of the batch runs net pool->block_model[b], the kernels stop at
+// the padded row count *pool->n_rows, and the head epilogue writes action / logits by env (the per-layer head included: no
+// categorical launch).
+template <bool GROUPED = false>
 static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams* p, const void* obs, const unsigned char* blob,
                                 __nv_bfloat16* scratch, float* logits, float* value, const ActArgs& act, const PoolArgs* pool = nullptr) {
     int32_t rc = BRL_OK;
@@ -983,8 +971,8 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
     __nv_bfloat16* buf_lo[2] = {scratch + 2 * act_elems, scratch + 3 * act_elems};
     if (fused_forward(p)) {
         uint32_t* ready = reinterpret_cast<uint32_t*>(scratch + 4 * act_elems);
-        rc = split ? launch_fused<true, GROUPED, DEVCOUNT>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
-                   : launch_fused<false, GROUPED, DEVCOUNT>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
+        rc = split ? launch_fused<true, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool)
+                   : launch_fused<false, GROUPED>(s, obs, blob, L, buf_hi, buf_lo, ready, logits, value, M, act, pool);
         if (rc != BRL_OK) return rc;
         return check_launch(who);
     }
@@ -1006,16 +994,16 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
             a.out_lo = split ? buf_lo[l & 1] : nullptr;
             // 128 x 256 tiles move fewer operand bytes per MMA (the L2 -> SM fill rate, ~64 B/clk, is what bounds
             // these 1-CTA tiles): measured faster for the single-product mode; the split mode runs 128 x 128 tiles
-            if (!split) rc = launch_layer<256, false, false, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            else if (l == 0) rc = launch_layer<128, false, true, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
-            else rc = launch_layer<128, true, true, false, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            if (!split) rc = launch_layer<256, false, false, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else if (l == 0) rc = launch_layer<128, false, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
+            else rc = launch_layer<128, true, true, false, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHidden, a, pool);
             in_hi = a.out_hi;
             in_lo = a.out_lo;
         } else {
             a.logits = GROUPED ? logits : lg;
             a.value = GROUPED ? nullptr : vl;
-            rc = split ? launch_layer<kHeadPad, true, true, true, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool)
-                       : launch_layer<kHeadPad, false, false, true, GROUPED, DEVCOUNT>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool);
+            rc = split ? launch_layer<kHeadPad, true, true, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool)
+                       : launch_layer<kHeadPad, false, false, true, GROUPED>(s, in_hi, in_lo, L.k_in[l], w_hi, w_lo, kHeadPad, a, pool);
         }
         if (rc != BRL_OK) return rc;
     }
@@ -1026,26 +1014,51 @@ static int32_t mlp_forward_impl(const char* who, cudaStream_t s, const BrlParams
                               act.row_index ? logits : nullptr);
 }
 
-// brl_policy_act_rows / brl_policy_act_grouped, whose buffers share the slots [0] obs, [1] net or pool, [2] scratch, [3] mask,
-// [4] action, [5] rows, [7] logits: gather the listed rows' observations (one 960-byte bf16 row per thread group) behind the
-// forward's scratch, run the forward on the compact batch, and let the head epilogue read mask[env] and write action[env] /
-// log_prob[env] / logits[env].  GROUPED: row -1 (a group's padding) gathers zeros; block_model = the net of each row block.
-template <bool GROUPED>
-static int32_t policy_act_listed(const char* who, cudaStream_t s, void** b, const BrlParams* p, ActArgs act,
-                                 const int32_t* block_model = nullptr) {
-    const int64_t n = p->n_envs;
-    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
-    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
+namespace brl {
+
+// ---- the grouped forward: brl_policy_act_grouped and the device loops of brl_duplicate_match / brl_evaluate_match -------------
+// Every env listed in rows[0, *n_rows) is forwarded by the net of its kGroupRows-row block (block_model) out of the pool of
+// `n_models` nets, and the head epilogue reads mask[env] and writes action[env] / logits[env] (`logits`: f32[total, 38] or NULL).
+// The padded row count *n_rows (brl_model_rows' offsets[M]) is read on the device only: the gather, the launches and their tensor
+// maps are sized for `capacity` rows, and the threads and row blocks past the count exit at once.  Row -1 (a group's padding)
+// gathers zeros and its outputs are dropped.  The path is fused_forward's rule on `capacity` and the BRL_F_TUNE_MLP_* bits of
+// `flags` (BRL_F_MLP_BF16 selects the single-product mode).
+int32_t launch_policy_grouped(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
+                              const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
+                              const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits) {
+    BrlParams p{};
+    p.n_envs = capacity;
+    p.flags = flags;
+    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(capacity));
     const int w = kObsDimM * 2 / 16;  // uint4 per bf16 observation row
-    k_gather_obs_rows<GROUPED><<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]),
-                                                                              static_cast<const int32_t*>(b[5]), gathered, n, w);
-    act.mask = static_cast<const uint8_t*>(b[3]);
-    act.action = static_cast<int32_t*>(b[4]);
-    act.row_index = static_cast<const int32_t*>(b[5]);
-    const PoolArgs pool{block_model, brl_mlp_pool_stride(), p->k_steps, act};
-    return mlp_forward_impl<GROUPED>(who, s, p, gathered, static_cast<const unsigned char*>(b[1]), reinterpret_cast<__nv_bfloat16*>(scratch),
-                                     static_cast<float*>(b[7]), nullptr, act, GROUPED ? &pool : nullptr);
+    k_gather_obs_rows_grouped<<<(unsigned)((capacity * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(obs), rows, gathered,
+                                                                                     n_rows, w);
+    ActArgs act{};
+    act.mask = mask;
+    act.action = action;
+    act.row_index = rows;
+    const PoolArgs pa{block_model, brl_mlp_pool_stride(), n_models, act, n_rows};
+    return mlp_forward_impl<true>("brl_policy_act_grouped", s, &p, gathered, pool, reinterpret_cast<__nv_bfloat16*>(scratch), logits,
+                                  nullptr, act, &pa);
 }
+
+// everything launch_policy_grouped sets up once per device -- the driver's tensor-map entry point, the kernels' shared-memory
+// attributes, the fused kernel's co-resident pair count -- done before a stream capture begins
+int32_t warm_policy_grouped(bool split) {
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "device match loop: cuTensorMapEncodeTiled not available from the driver");
+    int32_t rc;
+    if (split) {
+        if ((rc = layer_attr<128, false, true, false, true>()) || (rc = layer_attr<128, true, true, false, true>()) ||
+            (rc = layer_attr<kHeadPad, true, true, true, true>()))
+            return rc;
+        return fused_pairs<true, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
+    }
+    if ((rc = layer_attr<256, false, false, false, true>()) || (rc = layer_attr<kHeadPad, false, false, true, true>()))
+        return rc;
+    return fused_pairs<false, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
+}
+
+}  // namespace brl
 
 extern "C" {
 
@@ -1092,13 +1105,26 @@ int32_t brl_policy_act_rows(brl_stream_t stream, void** b, const void* opaque, s
     BRL_REQUIRE(b[5], "row_index");
     if (b[3] != nullptr && (reinterpret_cast<uintptr_t>(b[3]) & 1u)) return fail(BRL_E_BUFFER, "brl_policy_act_rows: mask is misaligned");
     if (b[7] != nullptr && (reinterpret_cast<uintptr_t>(b[7]) & 7u)) return fail(BRL_E_BUFFER, "brl_policy_act_rows: logits is misaligned");
+    // gather the listed rows' observations (one 960-byte bf16 row per thread group) behind the forward's scratch, run the forward
+    // on the compact batch, and let the head epilogue read mask[env] and write action[env] / log_prob[env] / logits[env]
+    const cudaStream_t s = (cudaStream_t)stream;
+    const int64_t n = p->n_envs;
+    unsigned char* scratch = static_cast<unsigned char*>(b[2]);
+    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(n));
+    const int w = kObsDimM * 2 / 16;  // uint4 per bf16 observation row
+    k_gather_obs_rows<<<(unsigned)((n * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(b[0]), static_cast<const int32_t*>(b[5]),
+                                                                       gathered, n, w);
     ActArgs act{};
+    act.mask = static_cast<const uint8_t*>(b[3]);
+    act.action = static_cast<int32_t*>(b[4]);
     act.log_prob = static_cast<float*>(b[6]);
     act.seed = p->seed;
     act.env_offset = p->env_offset;
     act.step = p->step;
     act.sample = (p->flags & BRL_F_SAMPLE) ? 1 : 0;
-    return policy_act_listed<false>("brl_policy_act_rows", (cudaStream_t)stream, b, p, act);
+    act.row_index = static_cast<const int32_t*>(b[5]);
+    return mlp_forward_impl("brl_policy_act_rows", s, p, gathered, static_cast<const unsigned char*>(b[1]),
+                            reinterpret_cast<__nv_bfloat16*>(scratch), static_cast<float*>(b[7]), nullptr, act);
 }
 
 int64_t brl_mlp_pool_stride(void) { return (int64_t)mlp_layout().total; }  // a multiple of 256: every section keeps its TMA alignment
@@ -1127,13 +1153,19 @@ int32_t brl_policy_act_grouped(brl_stream_t stream, void** b, const void* opaque
     BRL_REQUIRE(b[4], "action");
     BRL_REQUIRE(b[5], "rows");
     BRL_REQUIRE(b[6], "block_model");
+    // n_rows is typically offsets + M of brl_model_rows: one int32, so 4-byte alignment is all it needs
+    if (b[8] == nullptr) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: buffer 'n_rows' is NULL");
+    if (reinterpret_cast<uintptr_t>(b[8]) & 3u) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: n_rows is misaligned");
     if (b[3] != nullptr && (reinterpret_cast<uintptr_t>(b[3]) & 1u)) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: mask is misaligned");
     if (b[7] != nullptr && (reinterpret_cast<uintptr_t>(b[7]) & 7u)) return fail(BRL_E_BUFFER, "brl_policy_act_grouped: logits is misaligned");
     if (p->k_steps <= 0) return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: k_steps (the pool's model count) must be > 0");
     if (p->n_envs % kGroupRows != 0)
         return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: n_envs (padded rows) must be a multiple of %d", kGroupRows);
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_policy_act_grouped: sampling is not supported (argmax only)");
-    return policy_act_listed<true>("brl_policy_act_grouped", (cudaStream_t)stream, b, p, ActArgs{}, static_cast<const int32_t*>(b[6]));
+    return launch_policy_grouped((cudaStream_t)stream, p->flags, p->n_envs, p->k_steps, b[0], static_cast<const unsigned char*>(b[1]),
+                                 static_cast<unsigned char*>(b[2]), static_cast<const uint8_t*>(b[3]), static_cast<int32_t*>(b[4]),
+                                 static_cast<const int32_t*>(b[5]), static_cast<const int32_t*>(b[6]), static_cast<const int32_t*>(b[8]),
+                                 static_cast<float*>(b[7]));
 }
 
 int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -1168,48 +1200,3 @@ int32_t brl_policy_act(brl_stream_t stream, void** b, const void* opaque, size_t
 }
 
 }  // extern "C"
-
-namespace brl {
-
-// ---- the grouped forward of the device loops of brl_duplicate_match / brl_evaluate_match (brl_match.cu) ---------------------
-// brl_policy_act_grouped with the padded row count in device memory (`n_rows` = brl_model_rows' offsets[M]): the gather, the
-// launches and their tensor maps are sized for `capacity` rows, and the DEVCOUNT kernels stop at the count.  The caller picks the
-// path: `flags` holds BRL_F_TUNE_MLP_LAYERS or BRL_F_TUNE_MLP_FUSED (and BRL_F_MLP_BF16 for the single-product mode).  `logits`
-// (f32[n, 38] or NULL): the listed rows' logits, written by env as brl_policy_act_grouped's buffer [7].
-int32_t launch_policy_grouped_dev(cudaStream_t s, int32_t flags, int64_t capacity, int n_models, const void* obs,
-                                  const unsigned char* pool, unsigned char* scratch, const uint8_t* mask, int32_t* action,
-                                  const int32_t* rows, const int32_t* block_model, const int32_t* n_rows, float* logits) {
-    BrlParams p{};
-    p.n_envs = capacity;
-    p.flags = flags;
-    p.k_steps = n_models;
-    uint4* gathered = reinterpret_cast<uint4*>(scratch + brl_mlp_scratch_bytes(capacity));
-    const int w = kObsDimM * 2 / 16;
-    k_gather_obs_rows_dev<<<(unsigned)((capacity * w + 255) / 256), 256, 0, s>>>(static_cast<const uint4*>(obs), rows, gathered,
-                                                                                 n_rows, w);
-    ActArgs act{};
-    act.mask = mask;
-    act.action = action;
-    act.row_index = rows;
-    const PoolArgs pa{block_model, brl_mlp_pool_stride(), n_models, act, n_rows};
-    return mlp_forward_impl<true, true>("grouped forward (device count)", s, &p, gathered, pool, reinterpret_cast<__nv_bfloat16*>(scratch),
-                                        logits, nullptr, act, &pa);
-}
-
-// everything launch_policy_grouped_dev sets up once per device -- the driver's tensor-map entry point, the kernels'
-// shared-memory attributes, the fused kernel's co-resident pair count -- done before a stream capture begins
-int32_t warm_policy_grouped_dev(bool split) {
-    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "device match loop: cuTensorMapEncodeTiled not available from the driver");
-    int32_t rc;
-    if (split) {
-        if ((rc = layer_attr<128, false, true, false, true, true>()) || (rc = layer_attr<128, true, true, false, true, true>()) ||
-            (rc = layer_attr<kHeadPad, true, true, true, true, true>()))
-            return rc;
-        return fused_pairs<true, true, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
-    }
-    if ((rc = layer_attr<256, false, false, false, true, true>()) || (rc = layer_attr<kHeadPad, false, false, true, true, true>()))
-        return rc;
-    return fused_pairs<false, true, true>() > 0 ? BRL_OK : BRL_E_LAUNCH;
-}
-
-}  // namespace brl

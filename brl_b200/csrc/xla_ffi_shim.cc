@@ -72,7 +72,7 @@
     X(brl_sl_grad, "iisiioos") \
     X(brl_sl_eval, "iisiios") \
     X(brl_model_rows, "iiioooo") \
-    X(brl_policy_act_grouped, "iisixiix") \
+    X(brl_policy_act_grouped, "iisixiixi") \
     X(brl_match_stats_ranges, "iix") \
     X(brl_duplicate_match, "iiiiisoxooooooooooooo") \
     X(brl_evaluate_match, "iiisooxooooooooooooooooooo") \

@@ -556,21 +556,28 @@ def model_rows(current_player: torch.Tensor, done: Optional[torch.Tensor], env_m
 
 def policy_act_grouped(obs_bf16: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, mask: Optional[torch.Tensor],
                        action: torch.Tensor, rows: torch.Tensor, block_model: torch.Tensor,
-                       logits: Optional[torch.Tensor] = None, *, single_bf16: bool = False, tune: int = 0) -> None:
+                       logits: Optional[torch.Tensor] = None, *, n_rows: Optional[torch.Tensor] = None,
+                       single_bf16: bool = False, tune: int = 0) -> None:
     """`policy_act_rows` (masked argmax) for the padded, net-grouped `rows` of `model_rows`, net block_model[b] on rows
-    [256 b, 256 b + 256), all nets of `pool` (u8[M, mlp_pool_stride()]) in one forward.  rows / block_model must come from
-    `model_rows` with the same M (device data, not checked here)."""
+    [256 b, 256 b + 256), all nets of `pool` (u8[M, mlp_pool_stride()]) in one forward.  n_rows[0] is the padded row count
+    (`offsets[M:]` of `model_rows`), read on the device only: rows from n_rows[0] on are not read, and the call is sized
+    (and its launch path chosen) for rows.shape[0].  Without n_rows the rows end at the count (rows = rows[:offsets[M]]).
+    rows / block_model / n_rows must come from `model_rows` with the same M (device data, not checked here)."""
     n = rows.shape[0]
     if n == 0:
         return
     if obs_bf16.dtype != torch.bfloat16 or rows.dtype != torch.int32 or block_model.dtype != torch.int32:
         raise _lib.BrlError("policy_act_grouped needs a bf16 observation and int32 rows / block_model")
+    if n_rows is None:
+        n_rows = torch.full((1,), n, dtype=torch.int32, device=rows.device)
+    if not n_rows.is_cuda or n_rows.dtype != torch.int32 or n_rows.numel() < 1:
+        raise _lib.BrlError("policy_act_grouped: n_rows must be a CUDA int32 tensor holding the padded row count (offsets[M:])")
     if pool.dim() != 2 or pool.shape[1] != mlp_pool_stride() or pool.dtype != torch.uint8:
         raise _lib.BrlError("policy_act_grouped: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
     if scratch.numel() < _lib.load().brl_mlp_rows_scratch_bytes(n):
         raise _lib.BrlError("policy_act_grouped: scratch too small (ops.policy_grouped_scratch_bytes)")
     _call("brl_policy_act_grouped", [_ptr(obs_bf16), _ptr(pool), _ptr(scratch), _ptr(mask), _ptr(action), _ptr(rows),
-                                     _ptr(block_model), _ptr(logits)],
+                                     _ptr(block_model), _ptr(logits), _ptr(n_rows)],
           _params(n, k_steps=pool.shape[0], flags=(F_MLP_BF16 if single_bf16 else 0) | tune))
 
 

@@ -62,7 +62,7 @@
  *   brl_model_rows        the per-team net choice of every league match: live rows grouped by acting net
  *                                                      workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
  *   brl_policy_act_grouped  team{1,2}_forward_pass.apply + masked argmax of every match of a league, one forward over a
- *                         pool of nets                 workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
+ *                         pool of nets, row count read on the device   workspace/eval_selfplay_league.py ; src/evaluation.py:124-151
  *   brl_match_stats_ranges  brl_match_stats of every match of a league chunk   src/evaluation.py:199-201
  *   brl_duplicate_match   jax.jit(make_simple_duplicate_evaluate(...)) as one call: init, Table_info, the whole
  *                         lax.while_loop and the match sums   eval.py:53 ; src/evaluation.py:69-204
@@ -85,7 +85,7 @@ extern "C" {
 typedef struct CUstream_st *brl_stream_t; /* == cudaStream_t */
 #endif
 
-#define BRL_ABI_VERSION 2
+#define BRL_ABI_VERSION 3
 #define BRL_NUM_ACTIONS 38      /* 0 Pass, 1 X, 2 XX, 3..37 = 1C..7NT (src/duplicate.py:9-12) */
 #define BRL_OBS_DIM 480         /* ppo.py:241, wb5/utils.py:48-52 */
 #define BRL_NUM_PLAYERS 4
@@ -271,9 +271,10 @@ int32_t brl_team_rows(brl_stream_t, void **buffers, const void *opaque, size_t o
 
 /* ---- self-play league over a pool of M nets (workspace/eval_selfplay_league.py; each match src/evaluation.py:69-204) ----
  * All matches of the league run as one batch of envs.  The pool is M packed blobs (brl_mlp_pack) stacked
- * brl_mlp_pool_stride() bytes apart.  Every live env is forwarded by the net that acts there, with a one-host-read-per-step
- * loop: brl_model_rows groups the rows by net, the host reads offsets[M] (the padded row count; 0 = every env finished),
- * brl_policy_act_grouped runs all nets in one forward.  BrlParams.k_steps = M in both. */
+ * brl_mlp_pool_stride() bytes apart.  Every live env is forwarded by the net that acts there: brl_model_rows groups the rows
+ * by net and writes the padded row count offsets[M] to device memory, and brl_policy_act_grouped runs all nets in one forward
+ * that reads that count on the device, so a step needs no host read.  brl_duplicate_match plays a whole match this way.
+ * BrlParams.k_steps = M in both. */
 int64_t brl_mlp_pool_stride(void);
 /* rows a grouping of n_envs envs over M nets can need: each non-empty group is padded to 256 rows (one row tile) */
 int64_t brl_model_rows_capacity(int64_t n_envs, int64_t n_models);
@@ -287,13 +288,17 @@ int64_t brl_model_rows_capacity(int64_t n_envs, int64_t n_models);
  * An empty batch (n_envs = 0) zeroes counts / offsets when they are given. */
 int32_t brl_model_rows(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 /* brl_policy_act_rows with the net of each row block taken from the pool (masked argmax only; BRL_F_SAMPLE is an error).
- * n_envs = the padded row count offsets[M] of brl_model_rows; action and logits of the listed envs are written by env.
- * buffers: [0] in bf16 obs[total,480]  [1] in pool u8[M, brl_mlp_pool_stride()]  [2] scratch
- *          (brl_policy_grouped_scratch_bytes(total, M))  [3] in u8 mask[total,38] (NULL -> unmasked)  [4] out i32 action[total]
- *          [5] in i32 rows[n_envs]  [6] in i32 block_model[n_envs / 256]  [7] out f32 logits[total,38] (NULL ok)
- * params: n_envs (a multiple of 256), k_steps = M, flags BRL_F_MLP_BF16.
- * rows / block_model must be brl_model_rows' output for the same M: they are device data and not checked here; a block id
- * outside [0, M) is undefined behaviour. */
+ * The row count n_rows[0] (offsets[M] of brl_model_rows, e.g. a pointer to offsets + M) is read on the device only: the call
+ * is sized for n_envs rows, and the rows from n_rows[0] on are not read.  Action and logits of the listed envs are written by env.
+ * buffers: [0] in bf16 obs[total,480]  [1] in pool u8[M, brl_mlp_pool_stride()]  [2] scratch (brl_mlp_rows_scratch_bytes(n_envs),
+ *          = brl_policy_grouped_scratch_bytes(total, M) for the capacity)  [3] in u8 mask[total,38] (NULL -> unmasked)
+ *          [4] out i32 action[total]  [5] in i32 rows[n_envs]  [6] in i32 block_model[n_envs / 256]
+ *          [7] out f32 logits[total,38] (NULL ok)  [8] in i32 n_rows[1] (4-byte aligned)
+ * params: n_envs = the capacity of rows (a multiple of 256, e.g. brl_model_rows_capacity(total, M)), k_steps = M, flags
+ *         BRL_F_MLP_BF16 / BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED.  The path is brl_policy_act's rule on n_envs (one fused
+ *         launch from 4096 on, per-layer launches below), so n_envs = n_rows[0] runs the path of that batch size.
+ * rows / block_model / n_rows must be brl_model_rows' output for the same M, with n_rows[0] <= n_envs: they are device data and
+ * not checked here; a block id outside [0, M) or a count above n_envs is undefined behaviour. */
 int64_t brl_policy_grouped_scratch_bytes(int64_t n_envs, int64_t n_models);
 int32_t brl_policy_act_grouped(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 /* brl_match_stats over P = n_envs contiguous ranges (the matches of a league chunk), each entry exactly what brl_match_stats

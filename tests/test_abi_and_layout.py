@@ -25,7 +25,7 @@ def test_header_symbols_are_all_exported():
     for name in names:
         assert hasattr(L, name), f"{name} declared in include/brl_b200.h but not exported"
     assert set(_lib.ALL_SYMBOLS) == set(names)
-    assert L.brl_abi_version() == _lib.ABI_VERSION == 2
+    assert L.brl_abi_version() == _lib.ABI_VERSION == 3
 
 
 def test_params_struct_matches_header():

@@ -484,7 +484,8 @@ def test_grouped_forward_matches_each_nets_float64(sizes, tune, record_property)
     off = offsets.tolist()
     scratch = torch.empty(ops.policy_grouped_scratch_bytes(n, M), dtype=torch.uint8, device=DEV).fill_(0xFF)
     action, logits = torch.full((n,), -7, dtype=torch.int32, device=DEV), _nan(n, 38)
-    ops.policy_act_grouped(x, pool, scratch, mask, action, rows[:off[M]], block_model, logits, tune=tune)
+    ops.policy_act_grouped(x, pool, scratch, mask, action, rows[:off[M]], block_model, logits, n_rows=offsets[M:],
+                           tune=tune)
     assert bool(torch.isfinite(logits).all()) and bool((action >= 0).all()), "an env was not written"
     worst = 0.0
     for m in range(M):

@@ -85,7 +85,8 @@ def test_grouped_forward_equals_per_model_listed_forward(case, single_bf16):
     action = torch.full((n,), -5, dtype=torch.int32, device=DEV)
     logits = torch.full((n, 38), 7.0, dtype=torch.float32, device=DEV)
     scratch = torch.empty(ops.policy_grouped_scratch_bytes(n, M), dtype=torch.uint8, device=DEV)
-    ops.policy_act_grouped(obs, pool, scratch, mask, action, rows[:n_rows], block_model, logits, single_bf16=single_bf16)
+    ops.policy_act_grouped(obs, pool, scratch, mask, action, rows[:n_rows], block_model, logits, n_rows=offsets[M:],
+                           single_bf16=single_bf16)
     a_ref = torch.full((n,), -5, dtype=torch.int32, device=DEV)
     lg_ref = torch.full((n, 38), 7.0, dtype=torch.float32, device=DEV)
     for m in range(M):
@@ -97,7 +98,7 @@ def test_grouped_forward_equals_per_model_listed_forward(case, single_bf16):
     unlisted = torch.as_tensor(done_np, device=DEV) != 0
     assert bool((action[unlisted] == -5).all()) and bool((logits[unlisted] == 7.0).all())
     assert bool(mask[~unlisted].gather(1, action[~unlisted].long()[:, None]).all())
-    # the mask and logits are optional
+    # the mask and logits are optional, and without n_rows the rows end at the count
     a2 = torch.full((n,), -5, dtype=torch.int32, device=DEV)
     ops.policy_act_grouped(obs, pool, scratch, mask, a2, rows[:n_rows], block_model, single_bf16=single_bf16)
     assert torch.equal(a2, a_ref)
@@ -112,6 +113,62 @@ def test_grouped_forward_rejects_sampling():
     with pytest.raises(_lib.BrlError, match="sampling"):
         ops.policy_act_grouped(obs, pool, scratch, None, torch.zeros(4, dtype=torch.int32, device=DEV), rows,
                                torch.zeros(1, dtype=torch.int32, device=DEV), tune=_lib.F_SAMPLE)
+
+
+def test_grouped_forward_validates_the_row_count_tensor():
+    from brl_b200 import _lib, ops
+    rows, block_model = torch.zeros(256, dtype=torch.int32, device=DEV), torch.zeros(1, dtype=torch.int32, device=DEV)
+    obs = torch.zeros((4, 480), dtype=torch.bfloat16, device=DEV)
+    pool = torch.zeros((1, ops.mlp_pool_stride()), dtype=torch.uint8, device=DEV)
+    scratch = torch.empty(ops.policy_grouped_scratch_bytes(4, 1), dtype=torch.uint8, device=DEV)
+    for bad in (torch.full((1,), 256, dtype=torch.int64, device=DEV), torch.empty(0, dtype=torch.int32, device=DEV),
+                torch.full((1,), 256, dtype=torch.int32)):
+        with pytest.raises(_lib.BrlError, match="n_rows"):
+            ops.policy_act_grouped(obs, pool, scratch, None, torch.zeros(4, dtype=torch.int32, device=DEV), rows, block_model,
+                                   n_rows=bad)
+
+
+@pytest.mark.parametrize("single_bf16", [False, True])
+@pytest.mark.parametrize("tune", [FORCE_FUSED, FORCE_LAYERS], ids=["fused", "layers"])
+@pytest.mark.parametrize("case", [2, 3])
+def test_grouped_forward_sized_past_the_row_count_equals_the_call_sized_for_it(case, tune, single_bf16):
+    """The device match loops size the grouped forward for the grouping's capacity and leave the padded row count in device
+    memory.  A rows buffer longer than offsets[M], padded with -1, gives the actions and logits of the call whose rows end at
+    the count; so does one that lists finished envs past the count, which must not be forwarded."""
+    from brl_b200 import ops
+    from brl_b200.models import make_forward_pass
+    M, sizes = CASES[case]
+    player, done, env_models, _, done_np = _grouping(sizes, n_done=300, seed=case)
+    n = player.shape[0]
+    obs, mask = _obs_and_mask(n, seed=case + 3)
+    fp = make_forward_pass(precision="tc-bf16" if single_bf16 else "tc")
+    pool = ops.mlp_pack_pool([H.seeded_params(100 + m, DEV) for m in range(M)], fp.pack_into)
+    cap = ops.model_rows_capacity(n, M)
+    rows = torch.full((cap,), -7, dtype=torch.int32, device=DEV)
+    block_model = torch.full((cap // 256,), -7, dtype=torch.int32, device=DEV)
+    counts, offsets = torch.empty(M, dtype=torch.int32, device=DEV), torch.empty(M + 1, dtype=torch.int32, device=DEV)
+    ops.model_rows(player, done, env_models, rows, counts, offsets, block_model)
+    n_rows, long = int(offsets[M]), int(offsets[M]) + 16 * 256
+
+    def run(rows_buf, blocks_buf):
+        action = torch.full((n,), -5, dtype=torch.int32, device=DEV)
+        logits = torch.full((n, 38), 7.0, dtype=torch.float32, device=DEV)
+        ops.policy_act_grouped(obs, pool, ops.mlp_rows_scratch(rows_buf.shape[0], DEV), mask, action, rows_buf, blocks_buf,
+                               logits, n_rows=offsets[M:], single_bf16=single_bf16, tune=tune)
+        return action, logits
+
+    a_ref, lg_ref = run(rows[:n_rows], block_model[:n_rows // 256])
+    assert bool((a_ref >= 0).sum() == sum(sizes))
+    rows_long = torch.full((long,), -1, dtype=torch.int32, device=DEV)
+    rows_long[:n_rows] = rows[:n_rows]
+    blocks_long = torch.zeros(long // 256, dtype=torch.int32, device=DEV)   # valid net ids past the count
+    blocks_long[:n_rows // 256] = block_model[:n_rows // 256]
+    a, lg = run(rows_long, blocks_long)
+    assert torch.equal(a, a_ref) and torch.equal(lg, lg_ref)
+    finished = torch.nonzero(torch.as_tensor(done_np, device=DEV)).flatten().to(torch.int32)
+    rows_long[n_rows:] = finished.repeat(-(-(long - n_rows) // finished.shape[0]))[:long - n_rows]
+    a, lg = run(rows_long, blocks_long)
+    assert torch.equal(a, a_ref) and torch.equal(lg, lg_ref)
 
 
 def _script_matrices(M, imps):
@@ -231,9 +288,9 @@ def test_league_xla_symbols_equal_direct_ops_and_empty_batches_are_no_ops():
     scratch = torch.empty(ops.policy_grouped_scratch_bytes(n, M), dtype=torch.uint8, device=DEV)
     acts = [torch.full((n,), -5, dtype=torch.int32, device=DEV) for _ in range(2)]
     lgs = [torch.full((n, 38), 7.0, dtype=torch.float32, device=DEV) for _ in range(2)]
-    ops.policy_act_grouped(obs, pool, scratch, mask, acts[0], rows[:n_rows], block_model, lgs[0])
-    _call_xla("brl_policy_act_grouped", [obs, pool, scratch, mask, acts[1], rows[:n_rows].contiguous(), block_model, lgs[1]],
-              ops._params(n_rows, k_steps=M))
+    ops.policy_act_grouped(obs, pool, scratch, mask, acts[0], rows[:n_rows], block_model, lgs[0], n_rows=out[0][2][M:])
+    _call_xla("brl_policy_act_grouped", [obs, pool, scratch, mask, acts[1], rows[:n_rows].contiguous(), block_model, lgs[1],
+                                         out[0][2][M:]], ops._params(n_rows, k_steps=M))
     torch.cuda.synchronize()
     assert torch.equal(acts[0], acts[1]) and torch.equal(lgs[0], lgs[1])
     x = torch.arange(1000, device=DEV, dtype=torch.float32) % 7 - 3

@@ -72,12 +72,12 @@ def test_league_ops_validate_their_arguments_without_a_gpu():
         fn.restype, fn.argtypes = ctypes.c_int32, [ctypes.c_void_p, ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_size_t]
 
     def call(name, bufs, p, size=None):
-        arr = (ctypes.c_void_p * 8)(*bufs)
+        arr = (ctypes.c_void_p * 9)(*bufs)
         return getattr(L, name)(None, arr, ctypes.byref(p), ctypes.sizeof(p) if size is None else size)
 
     p = _lib.BrlParams(512, 0, 0, 0, 0, 0, 0, 3, 0.0, 0.0, 0.0, 0.0)   # n_envs, ..., k_steps = M
-    null = [None] * 8
-    fake = [4096] * 8   # aligned, never dereferenced: each check below fails first
+    null = [None] * 9
+    fake = [4096] * 9   # aligned, never dereferenced: each check below fails first
     for name in ("brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges"):
         assert call(name, null, p, 12) == -1 and b"BrlParams" in L.brl_last_error()
         assert call(name, null, p) == -2 and b"NULL" in L.brl_last_error()
@@ -85,8 +85,12 @@ def test_league_ops_validate_their_arguments_without_a_gpu():
     p0 = _lib.BrlParams(0, 0, 0, 0, 0, 0, 0, 3, 0.0, 0.0, 0.0, 0.0)
     for name in ("brl_policy_act_grouped", "brl_match_stats_ranges"):
         assert call(name, null, p0) == 0
-    bad = [4096, 4096, 4096, 4097, 4096, 4096, 4096, 4096]
+    bad = [4096, 4096, 4096, 4097, 4096, 4096, 4096, 4096, 4096]
     assert call("brl_policy_act_grouped", bad, p) == -2 and b"mask" in L.brl_last_error()
+    # n_rows (buffer 8) points at offsets[M]: one int32, 4-byte aligned is enough
+    assert call("brl_policy_act_grouped", fake[:8] + [None], p) == -2 and b"n_rows" in L.brl_last_error()
+    assert call("brl_policy_act_grouped", fake[:8] + [4098], p) == -2 and b"n_rows" in L.brl_last_error()
+    assert call("brl_policy_act_grouped", fake[:3] + [4097] + fake[4:8] + [4100], p) == -2 and b"mask" in L.brl_last_error()
     pk = _lib.BrlParams(512, 0, 0, 0, 0, 0, 0, 0, 0.0, 0.0, 0.0, 0.0)
     assert call("brl_policy_act_grouped", fake, pk) == -1 and b"model count" in L.brl_last_error()
     assert call("brl_model_rows", fake, pk) == -1 and b"model count" in L.brl_last_error()
@@ -96,7 +100,7 @@ def test_league_ops_validate_their_arguments_without_a_gpu():
     assert call("brl_policy_act_grouped", fake, ps) == -1 and b"sampling" in L.brl_last_error()
     for name in ("brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges"):
         assert L.brl_xla_layout(name.encode()) is not None
-    assert L.brl_xla_layout(b"brl_policy_act_grouped") == b"iisixiix"
+    assert L.brl_xla_layout(b"brl_policy_act_grouped") == b"iisixiixi"
 
 
 def test_league_ops_are_bound_lazily():
