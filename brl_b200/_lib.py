@@ -15,7 +15,7 @@ from . import build as _build
 # eagerly moved the interpreter's garbage-collection schedule in bench.py so that its rollout leg measured 8 % slower on a
 # B200 (1000 W), with identical device code and identical timings under gc.disable().
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
-            "brl_duplicate_match", "brl_evaluate_match")
+            "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -31,7 +31,8 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_xla_layout", "brl_xla_unreported_failures", "brl_eval_num_sums",
         "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset",
         "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes",
-        "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes")
+        "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes",
+        "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 
@@ -91,6 +92,13 @@ class BrlPpoParams(C.Structure):
 class BrlAdamParams(C.Structure):
     _fields_ = [("n", C.c_int64), ("step", C.c_int32), ("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float),
                 ("eps", C.c_float), ("max_grad_norm", C.c_float)]
+
+
+class BrlPpoGroupedParams(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("n_learners", C.c_int32), ("flags", C.c_int32), ("reserved", C.c_int32), ("pad", C.c_int32)]
+
+
+MAX_LEARNERS = 64  # include/brl_b200.h BRL_MAX_LEARNERS
 
 
 class BrlSlParams(C.Structure):

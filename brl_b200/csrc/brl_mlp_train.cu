@@ -63,6 +63,10 @@ __host__ __device__ inline TrainBlob train_blob() {
     return T;
 }
 
+// row stride of a learner's flat parameters / gradients / moments in a population's [K, stride] buffers: 256-byte rows keep
+// every learner's float4 accesses aligned
+__host__ __device__ inline size_t param_stride() { return (flat_layout().total + 63) & ~(size_t)63; }
+
 // ---- optimizer step + re-pack in one pass (or the pack alone) -----------------------------------------------------
 // optax.chain(clip_by_global_norm, adam(eps)) over the flat buffer exactly as brl_adam_apply (csrc/brl_ppo.cu), and in the
 // same pass the refreshed parameter goes out as bf16 hi / lo (weights, same [in, out] orientation) or fp32 (biases) into the
@@ -80,10 +84,13 @@ struct AdamPackArgs {
     TrainBlob T;
 };
 
-__device__ __forceinline__ float adam_elem(const AdamPackArgs& a, float p, float g, float& m, float& v, float scale) {
+template <class A>  // AdamPackArgs, or a learner's AdamLearnerView
+__device__ __forceinline__ float adam_elem(const A& a, float p, float g, float& m, float& v, float scale) {
+    // the roundings spelled out: which products the compiler contracts into an FMA depends on where the scalars live
+    // (parameter space or registers), and every instantiation must give the bits of brl_mlp_adam_step
     const float gi = g * scale;
-    m = a.b1 * m + (1.0f - a.b1) * gi;
-    v = a.b2 * v + (1.0f - a.b2) * gi * gi;
+    m = __fmaf_rn(m, a.b1, __fmul_rn(gi, 1.0f - a.b1));
+    v = __fmaf_rn(v, a.b2, __fmul_rn(gi, __fmul_rn(gi, 1.0f - a.b2)));
     return p - a.lr * (m / a.bc1) / (sqrtf(v / a.bc2) + a.eps);
 }
 __device__ __forceinline__ void split_pair(float v0, float v1, uint32_t& hi, uint32_t& lo) {
@@ -92,10 +99,8 @@ __device__ __forceinline__ void split_pair(float v0, float v1, uint32_t& hi, uin
     lo = pack_bf16x2(v0 - __low2float(h), v1 - __high2float(h));
 }
 
-template <bool ADAM>
-__global__ void __launch_bounds__(256) k_adam_pack(const __grid_constant__ AdamPackArgs a) {
-    pdl_trigger();
-    pdl_wait();
+template <bool ADAM, class A>  // AdamPackArgs, or a learner's AdamLearnerView
+__device__ __forceinline__ void adam_pack_body(const A& a) {
     float scale = 1.0f;
     if (ADAM && a.max_norm > 0.0f) {  // optax.clip_by_global_norm: g * (max_norm / norm) only when norm >= max_norm
         const float norm = (float)sqrt(*a.sumsq);
@@ -157,6 +162,46 @@ __global__ void __launch_bounds__(256) k_adam_pack(const __grid_constant__ AdamP
         }
     }
 }
+template <bool ADAM>
+__global__ void __launch_bounds__(256) k_adam_pack(const __grid_constant__ AdamPackArgs a) {
+    pdl_trigger();
+    pdl_wait();
+    adam_pack_body<ADAM, AdamPackArgs>(a);
+}
+
+// the optimizer steps of K learners (brl_mlp_adam_step_grouped), blockIdx.y = learner: learner k's params / grads / m / v
+// lie k * param_stride() floats after learner 0's, its blob k * T.total bytes, its |g|^2 k * sumsq_stride doubles
+struct AdamLearner {
+    float max_norm, lr, b1, b2, eps, bc1, bc2;
+};
+struct GroupedAdamArgs {
+    AdamPackArgs a;  // learner 0's buffers
+    long long sumsq_stride;
+    AdamLearner l[BRL_MAX_LEARNERS];
+};
+// learner k's view of GroupedAdamArgs: its own pointers and scalars; the layouts stay in the parameter space (a local copy of
+// their arrays, indexed at run time, would live in local memory)
+struct AdamLearnerView {
+    float* p;
+    const float* g;
+    float* m;
+    float* v;
+    const double* sumsq;
+    unsigned char* blob;
+    float max_norm, lr, b1, b2, eps, bc1, bc2;
+    const FlatLayout& F;
+    const TrainBlob& T;
+};
+__global__ void __launch_bounds__(256) k_adam_pack_grouped(const __grid_constant__ GroupedAdamArgs g) {
+    pdl_trigger();
+    pdl_wait();
+    const int k = blockIdx.y;
+    const size_t n = param_stride() * k;
+    const AdamLearner& l = g.l[k];
+    const AdamLearnerView a{g.a.p + n, g.a.g + n, g.a.m + n, g.a.v + n, g.a.sumsq + k * g.sumsq_stride, g.a.blob + k * g.a.T.total,
+                            l.max_norm, l.lr, l.b1, l.b2, l.eps, l.bc1, l.bc2, g.a.F, g.a.T};
+    adam_pack_body<true, AdamLearnerView>(a);
+}
 
 // ---- per-minibatch scratch -------------------------------------------------------------------------------
 constexpr int kMaxOps = 9;  // GEMMs of one fused launch (forward: 5, backward: 9)
@@ -208,11 +253,9 @@ template <>
 __device__ __forceinline__ uint16_t obs_bits<__nv_bfloat16>(__nv_bfloat16 v) { return *reinterpret_cast<uint16_t*>(&v); }
 
 template <class T>
-__global__ void __launch_bounds__(256) k_gather_obs(const T* __restrict__ obs, const int32_t* __restrict__ index, int64_t B,
-                                                    uint16_t* __restrict__ out) {
+__device__ __forceinline__ void gather_obs_body(const T* __restrict__ obs, const int32_t* __restrict__ index, int64_t B,
+                                                uint16_t* __restrict__ out) {
     // 8 consecutive observation bits per thread: one 128-bit store
-    pdl_trigger();
-    pdl_wait();
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= B * (kObsDimM / 8)) return;
     const int64_t b = i / (kObsDimM / 8);
@@ -222,6 +265,23 @@ __global__ void __launch_bounds__(256) k_gather_obs(const T* __restrict__ obs, c
 #pragma unroll
     for (int k = 0; k < 4; ++k) w[k] = (uint32_t)obs_bits<T>(src[2 * k]) | ((uint32_t)obs_bits<T>(src[2 * k + 1]) << 16);
     *reinterpret_cast<uint4*>(out + b * kObsDimM + c) = make_uint4(w[0], w[1], w[2], w[3]);
+}
+template <class T>
+__global__ void __launch_bounds__(256) k_gather_obs(const T* __restrict__ obs, const int32_t* __restrict__ index, int64_t B,
+                                                    uint16_t* __restrict__ out) {
+    pdl_trigger();
+    pdl_wait();
+    gather_obs_body<T>(obs, index, B, out);
+}
+// K learners (blockIdx.y): learner k's observation and index from row k of the trajectory table, its rows to out + k * stride
+template <class T>
+__global__ void __launch_bounds__(256) k_gather_obs_grouped(const long long* __restrict__ traj, int64_t B, uint16_t* out,
+                                                            long long out_stride) {
+    pdl_trigger();
+    pdl_wait();
+    const long long* t = traj + 8 * blockIdx.y;
+    gather_obs_body<T>(reinterpret_cast<const T*>(t[0]), reinterpret_cast<const int32_t*>(t[1]), B,
+                       reinterpret_cast<uint16_t*>(reinterpret_cast<char*>(out) + blockIdx.y * out_stride));
 }
 
 // bias gradients: db[c] = sum_b dz[b, c].  Hidden layers: column sums of dz (hi + lo); a block owns 64 columns of one
@@ -239,19 +299,19 @@ struct BiasArgs {
     GramArgs gram;         // deferred spectral-norm statistic: its serial tail runs in one spare block (n_gram partials; 0 = none)
     int n_gram;
 };
-__device__ __forceinline__ void bias_sumsq(const BiasArgs& a, float v) {  // called by whole warps
+template <class A>  // BiasArgs, or a learner's BiasLearnerView
+__device__ __forceinline__ void bias_sumsq(const A& a, float v) {  // called by whole warps
     if (a.sumsq == nullptr) return;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     if ((threadIdx.x & 31) == 0) atomicAdd(a.sumsq, (double)v);
 }
-__global__ void __launch_bounds__(1024) k_bias_grad(const __grid_constant__ BiasArgs a) {
+template <class A>  // BiasArgs, or a learner's BiasLearnerView
+__device__ __forceinline__ void bias_grad_body(const A& a) {
     // a block either sums bias columns (red) or runs the Gram tail (GramSmem): one shared buffer for both
     constexpr size_t kSmemBytes = sizeof(GramSmem) > sizeof(float) * 32 * 65 ? sizeof(GramSmem) : sizeof(float) * 32 * 65;
     __shared__ __align__(16) unsigned char smem_raw[kSmemBytes];
     float (*red)[65] = reinterpret_cast<float (*)[65]>(smem_raw);
-    pdl_trigger();
-    pdl_wait();
     const int tid = threadIdx.x, rg = tid >> 5, cp = tid & 31;  // 32 row groups x 32 column pairs
     const int blocks_per_layer = kHidden / 64;
     if ((int)blockIdx.x > 4 * blocks_per_layer) {
@@ -300,6 +360,62 @@ __global__ void __launch_bounds__(1024) k_bias_grad(const __grid_constant__ Bias
             bias_sumsq(a, tot * tot);
         }
     }
+}
+__global__ void __launch_bounds__(1024) k_bias_grad(const __grid_constant__ BiasArgs a) {
+    pdl_trigger();
+    pdl_wait();
+    bias_grad_body<BiasArgs>(a);
+}
+// K learners (blockIdx.y), every learner's grid with the spare block; `a` holds learner 0's buffers.  The spare block runs
+// learner k's deferred Gram tail when its illegal_l2_coef is 0 and the statistic is asked for.
+struct GroupedBiasArgs {
+    BiasArgs a;
+    const long long* traj;   // [K][8] trajectory table (index, mask of the Gram tail)
+    const float* coefs;      // [K][4] loss coefficients (illegal_l2_coef: column 3)
+    const float* logits;     // learner 0's forward logits
+    float* stats;            // [K][8]
+    unsigned char* acc;      // [K][BRL_PPO_SCRATCH_BYTES]
+    long long sc_stride;     // bytes
+    int illegal_stat, n_gram;
+};
+// learner k's view of GroupedBiasArgs (as AdamLearnerView: the layout and the dz pointers stay in the parameter space)
+struct ShiftedRows {  // learner 0's per-layer pointers, read as learner k's
+    const __nv_bfloat16* const* base;
+    long long off;
+    __device__ __forceinline__ const __nv_bfloat16* operator[](int l) const {
+        return reinterpret_cast<const __nv_bfloat16*>(reinterpret_cast<const char*>(base[l]) + off);
+    }
+};
+struct BiasLearnerView {
+    ShiftedRows hi, lo;
+    const float* dlogits;
+    const float* dvalue;
+    float* grads;
+    double* sumsq;
+    int64_t B;
+    const FlatLayout& F;
+    GramArgs gram;
+    int n_gram;
+};
+__global__ void __launch_bounds__(1024) k_bias_grad_grouped(const __grid_constant__ GroupedBiasArgs g) {
+    pdl_trigger();
+    pdl_wait();
+    const int k = blockIdx.y;
+    const long long off = k * g.sc_stride;
+    auto sc = [&](auto* p) { return (decltype(p))((const char*)p + off); };
+    unsigned char* acc = g.acc + (size_t)k * BRL_PPO_SCRATCH_BYTES;
+    GramArgs gram{};
+    int n_gram = 0;
+    if ((int)blockIdx.x > 4 * (kHidden / 64)) {
+        if (!g.illegal_stat || g.coefs[4 * k + 3] != 0.0f) return;
+        const long long* t = g.traj + 8 * k;
+        gram = gram_args_at(sc(g.logits), reinterpret_cast<const int32_t*>(t[1]), reinterpret_cast<const uint8_t*>(t[2]), g.a.B, acc,
+                            g.stats + 8 * k + 6);
+        n_gram = g.n_gram;
+    }
+    const BiasLearnerView a{{g.a.hi, off}, {g.a.lo, off}, sc(g.a.dlogits), sc(g.a.dvalue), g.a.grads + k * param_stride(),
+                            reinterpret_cast<double*>(acc) + 14, g.a.B, g.a.F, gram, n_gram};
+    bias_grad_body<BiasLearnerView>(a);
 }
 
 // ---- the GEMM ---------------------------------------------------------------------------------------------
@@ -469,6 +585,37 @@ struct FusedTrainArgs {
     uint32_t* ready;         // [n_ops][nmb + 1]: per-row-block counters, then the op's total
     unsigned long long* trace;  // NULL, or [n_tiles][8] time stamps: dep wait begin / end, loads issued, first MMA, last MMA issued, accumulator seen, published
 };
+// The same launch for K learners (brl_ppo_grad_grouped).  Every op's tensor maps carry a trailing learner coordinate, and
+// its pointers are learner 0's: learner k's scratch, blob, gradient and |g|^2 lie k strides further.  Op o's tile range
+// holds the K learners' tiles of that op back to back (op.g.n_tiles is ONE learner's count), so a learner's chain waits
+// are filled by the other learners' tiles of the same op.  Counters: ready[(o * K + k) * (nmb + 1) + row block].
+struct GroupedTrainArgs {
+    FusedTrainArgs f;
+    int K;
+    long long sc_stride, blob_stride;  // bytes
+    long long grad_stride;             // floats
+    long long sumsq_stride;            // doubles
+};
+template <bool GROUPED>
+using TrainArgsT = std::conditional_t<GROUPED, GroupedTrainArgs, FusedTrainArgs>;
+__device__ __forceinline__ const FusedTrainArgs& fused_of(const FusedTrainArgs& a) { return a; }
+__device__ __forceinline__ const FusedTrainArgs& fused_of(const GroupedTrainArgs& a) { return a.f; }
+
+// learner k's epilogue arguments: every output pointer moved by its buffer's stride
+__device__ __forceinline__ GemmArgs learner_gemm(const GroupedTrainArgs& a, const GemmArgs& g, int k) {
+    GemmArgs r = g;
+    auto sc = [&](auto* p) { return p ? (decltype(p))((const char*)p + k * a.sc_stride) : p; };
+    r.out_hi = sc(g.out_hi);
+    r.out_lo = sc(g.out_lo);
+    r.relu_src = sc(g.relu_src);
+    r.logits = sc(g.logits);
+    r.value = sc(g.value);
+    r.bias = g.bias ? reinterpret_cast<const float*>(reinterpret_cast<const char*>(g.bias) + k * a.blob_stride) : nullptr;
+    r.c = g.c ? g.c + k * a.grad_stride : nullptr;
+    r.c2 = g.c2 ? g.c2 + k * a.grad_stride : nullptr;
+    r.sumsq = g.sumsq ? g.sumsq + k * a.sumsq_stride : nullptr;
+    return r;
+}
 
 // FBN = tile width of the fused launches: 64 keeps the most tiles in flight, 128 moves a third fewer operand bytes from
 // L2 per FLOP (the measured bound at minibatch sizes) and relies on tiles of different ops to fill the SMs.
@@ -496,8 +643,9 @@ __device__ __forceinline__ int fused_find_op(const FusedTrainArgs& a, int tile) 
     return o;
 }
 
-template <int kFBN>
-__global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_constant__ FusedTrainArgs a) {
+template <int kFBN, bool GROUPED>
+__global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_constant__ TrainArgsT<GROUPED> ga) {
+    const FusedTrainArgs& a = fused_of(ga);
     using Cfg = FusedTrainCfg<kFBN>;
     constexpr int S = Cfg::kStages;
     // The main loop is bound by the shared-memory port (TMA writes + the operand reads of the SS-mode MMAs, DESIGN.md), so
@@ -537,13 +685,16 @@ __global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_con
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 const int o = fused_find_op(a, tile);
                 const FusedOp& op = a.op[o];
-                const int r = tile - op.tile0;
+                int r = tile - op.tile0, k = 0;
+                if constexpr (GROUPED) { k = r / op.g.n_tiles; r -= k * op.g.n_tiles; }
                 const int mb = r / op.g.n_tiles_n, m0 = mb * kBM, n0 = (r % op.g.n_tiles_n) * kFBN;
                 const bool split_a = op.split_a != 0, a_mn = op.a_mn != 0, w_mn = op.w_mn != 0;
                 const uint32_t tx = Cfg::kABytes * (split_a ? 2u : 1u) + 2u * Cfg::kWBytes;
                 trace_stamp(a, tile, 0);
                 if (op.dep >= 0) {
-                    const uint32_t* flag = a.ready + (size_t)op.dep * (a.nmb + 1) + (op.dep_all ? a.nmb : mb);
+                    size_t counter = (size_t)op.dep;
+                    if constexpr (GROUPED) counter = counter * ga.K + k;
+                    const uint32_t* flag = a.ready + counter * (a.nmb + 1) + (op.dep_all ? a.nmb : mb);
                     uint32_t v = 0;
                     for (uint32_t spin = 0;; ++spin) {
                         asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
@@ -561,17 +712,31 @@ __global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_con
                     const uint32_t sa = base + s * Cfg::kStageBytes;
                     const uint32_t sw = sa + 2 * Cfg::kABytes;
                     // K-major operand: {64 k, rows (, hi / lo)}; MN-major: {64 features, 64 k rows, 64-feature chunks, hi / lo}
-                    if (!a_mn) {
-                        if (split_a) tma_load_3d(sa, &op.a, full_bar(s), kb * kBK, m0, 0);
-                        else tma_load_2d(sa, &op.a, full_bar(s), kb * kBK, m0);
-                    } else if (split_a) {
-                        tma_load_4d(sa, &op.a, full_bar(s), 0, kb * kBK, m0 / 64, 0);
-                    } else {
+                    if constexpr (!GROUPED) {
+                        if (!a_mn) {
+                            if (split_a) tma_load_3d(sa, &op.a, full_bar(s), kb * kBK, m0, 0);
+                            else tma_load_2d(sa, &op.a, full_bar(s), kb * kBK, m0);
+                        } else if (split_a) {
+                            tma_load_4d(sa, &op.a, full_bar(s), 0, kb * kBK, m0 / 64, 0);
+                        } else {
 #pragma unroll
-                        for (int j = 0; j < kBM / 64; ++j) tma_load_2d(sa + j * kMnBox, &op.a, full_bar(s), m0 + 64 * j, kb * kBK);
+                            for (int j = 0; j < kBM / 64; ++j) tma_load_2d(sa + j * kMnBox, &op.a, full_bar(s), m0 + 64 * j, kb * kBK);
+                        }
+                        if (!w_mn) tma_load_3d(sw, &op.w, full_bar(s), kb * kBK, n0, 0);
+                        else tma_load_4d(sw, &op.w, full_bar(s), 0, kb * kBK, n0 / 64, 0);
+                    } else {  // the same boxes, one more (learner) coordinate
+                        if (!a_mn) {
+                            if (split_a) tma_load_4d(sa, &op.a, full_bar(s), kb * kBK, m0, 0, k);
+                            else tma_load_3d(sa, &op.a, full_bar(s), kb * kBK, m0, k);
+                        } else if (split_a) {
+                            tma_load_5d(sa, &op.a, full_bar(s), 0, kb * kBK, m0 / 64, 0, k);
+                        } else {
+#pragma unroll
+                            for (int j = 0; j < kBM / 64; ++j) tma_load_3d(sa + j * kMnBox, &op.a, full_bar(s), m0 + 64 * j, kb * kBK, k);
+                        }
+                        if (!w_mn) tma_load_4d(sw, &op.w, full_bar(s), kb * kBK, n0, 0, k);
+                        else tma_load_5d(sw, &op.w, full_bar(s), 0, kb * kBK, n0 / 64, 0, k);
                     }
-                    if (!w_mn) tma_load_3d(sw, &op.w, full_bar(s), kb * kBK, n0, 0);
-                    else tma_load_4d(sw, &op.w, full_bar(s), 0, kb * kBK, n0 / 64, 0);
                 }
                 trace_stamp(a, tile, 2);
             }
@@ -618,7 +783,8 @@ __global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_con
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++j) {
             const int o = fused_find_op(a, tile);
             const FusedOp& op = a.op[o];
-            const int r = tile - op.tile0;
+            int r = tile - op.tile0, k = 0;
+            if constexpr (GROUPED) { k = r / op.g.n_tiles; r -= k * op.g.n_tiles; }
             const int mb = r / op.g.n_tiles_n, m0 = mb * kBM, n0 = (r % op.g.n_tiles_n) * kFBN;
             const uint32_t buf = j & 1u;
             mbar_wait(tmem_full_bar(buf), (j >> 1) & 1u);
@@ -627,16 +793,22 @@ __global__ void __launch_bounds__(kMlpThreads, 1) k_train_fused(const __grid_con
             const int row = m0 + q * 32 + lane;
             const uint32_t t_row = tmem_acc + buf * kBufCols + ((uint32_t)(q * 32) << 16);
             const bool row_ok = row < op.g.M;
-            if (op.epi == kEpiFwd) epilogue_act_row<kEpiFwd>(t_row, kFBN, n0, row, row_ok, op.g, (uint32_t)kFBN);
-            else if (op.epi == kEpiDgrad) epilogue_act_row<kEpiDgrad>(t_row, kFBN, n0, row, row_ok, op.g, (uint32_t)kFBN);
-            else if (op.epi == kEpiWgrad) epilogue_wgrad_row<kFBN>(t_row, n0, row, row_ok, op.g, (uint32_t)kFBN);
-            else epilogue_head_row2(t_row, (uint32_t)kFBN, op.g.bias + n0, row_ok, op.g.logits + (size_t)row * 38, op.g.value + row);
+            auto epilogue = [&](const GemmArgs& g) {
+                if (op.epi == kEpiFwd) epilogue_act_row<kEpiFwd>(t_row, kFBN, n0, row, row_ok, g, (uint32_t)kFBN);
+                else if (op.epi == kEpiDgrad) epilogue_act_row<kEpiDgrad>(t_row, kFBN, n0, row, row_ok, g, (uint32_t)kFBN);
+                else if (op.epi == kEpiWgrad) epilogue_wgrad_row<kFBN>(t_row, n0, row, row_ok, g, (uint32_t)kFBN);
+                else epilogue_head_row2(t_row, (uint32_t)kFBN, g.bias + n0, row_ok, g.logits + (size_t)row * 38, g.value + row);
+            };
+            if constexpr (GROUPED) epilogue(learner_gemm(ga, op.g, k));
+            else epilogue(op.g);
             tc_fence_before();
             __syncwarp();  // orders the other lanes' stores before lane 0's fence (the grid-barrier idiom: sync, one fence, one atomic)
             if (lane == 0) {
                 asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tmem_empty_bar(buf)) : "memory");
                 __threadfence();  // cumulative: the warp's output rows are visible GPU-wide before the counts below
-                uint32_t* cnt = a.ready + (size_t)o * (a.nmb + 1);
+                size_t counter = (size_t)o;
+                if constexpr (GROUPED) counter = counter * ga.K + k;
+                uint32_t* cnt = a.ready + counter * (a.nmb + 1);
                 atomicAdd(cnt + mb, 1u);
                 atomicAdd(cnt + a.nmb, 1u);
                 if (q == 0) trace_stamp(a, tile, 6);
@@ -659,35 +831,65 @@ struct OpSpec {
     int epi;
     GemmArgs g;
     int dep, dep_all;
+    long long a_stride, w_stride;  // grouped launch: bytes from learner k's operand to learner k + 1's
 };
 
-template <int kFBN>
+// the K learners of a grouped launch and the strides between their buffers
+struct GroupSpec {
+    int K;
+    long long sc_stride, blob_stride, grad_stride, sumsq_stride;
+};
+
+template <int kFBN, bool GROUPED = false>
 static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, int nmb, uint32_t* ready, unsigned long long* trace,
-                                const char* what) {
+                                const char* what, const GroupSpec* grp = nullptr) {
     using Cfg = FusedTrainCfg<kFBN>;
-    FusedTrainArgs fa{};
+    TrainArgsT<GROUPED> ga{};
+    FusedTrainArgs* fa_ptr;
+    if constexpr (GROUPED) fa_ptr = &ga.f;
+    else fa_ptr = &ga;
+    FusedTrainArgs& fa = *fa_ptr;
+    const int K = GROUPED ? grp->K : 1;
     int tiles = 0;
     for (int i = 0; i < n_ops; ++i) {
         const OpSpec& o = ops[i];
         FusedOp& f = fa.op[i];
+        // a grouped map has one more dimension, the learner, `stride` bytes apart
+        auto map_nd = [&](CUtensorMap* m, const void* ptr, int rank, uint64_t* dims, uint64_t* str, uint32_t* box, long long stride) {
+            if (GROUPED) {
+                dims[rank] = (uint64_t)K;
+                str[rank - 1] = (uint64_t)stride;
+                box[rank] = 1;
+                ++rank;
+            }
+            return make_map_nd(m, ptr, rank, dims, str, box);
+        };
         // (hi, lo) pair of one operand as a single map; feat = the operand's M / N extent, pitch in elements
-        auto pair_map = [&](CUtensorMap* m, const void* hi, const void* lo, bool mn, int feat, int pitch, uint32_t box_feat) {
+        auto pair_map = [&](CUtensorMap* m, const void* hi, const void* lo, bool mn, int feat, int pitch, uint32_t box_feat, long long stride) {
             if (static_cast<const char*>(lo) <= static_cast<const char*>(hi)) return false;  // the trailing dimension steps hi -> lo
             const uint64_t gap = (uint64_t)(static_cast<const char*>(lo) - static_cast<const char*>(hi));
             if (!mn) {  // K-major: [feat, k_cols]
-                const uint64_t dims[3] = {(uint64_t)o.k_cols, (uint64_t)feat, 2}, str[2] = {(uint64_t)pitch * 2, gap};
-                const uint32_t box[3] = {(uint32_t)kBK, box_feat, 2};
-                return make_map_nd(m, hi, 3, dims, str, box);
+                uint64_t dims[5] = {(uint64_t)o.k_cols, (uint64_t)feat, 2}, str[4] = {(uint64_t)pitch * 2, gap};
+                uint32_t box[5] = {(uint32_t)kBK, box_feat, 2};
+                return map_nd(m, hi, 3, dims, str, box, stride);
             }
             // MN-major: [k_cols, feat], features in chunks of 64
-            const uint64_t dims[4] = {64, (uint64_t)o.k_cols, (uint64_t)((feat + 63) / 64), 2}, str[3] = {(uint64_t)pitch * 2, 128, gap};
-            const uint32_t box[4] = {64, (uint32_t)kBK, box_feat / 64, 2};
-            return make_map_nd(m, hi, 4, dims, str, box);
+            uint64_t dims[5] = {64, (uint64_t)o.k_cols, (uint64_t)((feat + 63) / 64), 2}, str[4] = {(uint64_t)pitch * 2, 128, gap};
+            uint32_t box[5] = {64, (uint32_t)kBK, box_feat / 64, 2};
+            return map_nd(m, hi, 4, dims, str, box, stride);
         };
-        bool ok = pair_map(&f.w, o.w_hi, o.w_lo, o.w_mn != 0, o.n_rows, o.ldb, kFBN);
-        if (ok && o.a_lo) ok = pair_map(&f.a, o.a_hi, o.a_lo, o.a_mn != 0, o.m_rows, o.lda, kBM);
-        else if (ok) ok = o.a_mn ? make_map(&f.a, o.a_hi, (uint64_t)o.k_cols, (uint64_t)o.m_rows, (uint64_t)o.lda, 64)
-                                 : make_map(&f.a, o.a_hi, (uint64_t)o.m_rows, (uint64_t)o.k_cols, (uint64_t)o.lda, kBM);
+        bool ok = pair_map(&f.w, o.w_hi, o.w_lo, o.w_mn != 0, o.n_rows, o.ldb, kFBN, o.w_stride);
+        if (ok && o.a_lo) {
+            ok = pair_map(&f.a, o.a_hi, o.a_lo, o.a_mn != 0, o.m_rows, o.lda, kBM, o.a_stride);
+        } else if (ok && !GROUPED) {
+            ok = o.a_mn ? make_map(&f.a, o.a_hi, (uint64_t)o.k_cols, (uint64_t)o.m_rows, (uint64_t)o.lda, 64)
+                        : make_map(&f.a, o.a_hi, (uint64_t)o.m_rows, (uint64_t)o.k_cols, (uint64_t)o.lda, kBM);
+        } else if (ok) {  // make_map's boxes plus the learner dimension
+            const uint64_t rows = o.a_mn ? (uint64_t)o.k_cols : (uint64_t)o.m_rows, cols = o.a_mn ? (uint64_t)o.m_rows : (uint64_t)o.k_cols;
+            uint64_t dims[5] = {cols, rows}, str[4] = {(uint64_t)o.lda * 2};
+            uint32_t box[5] = {(uint32_t)kBK, o.a_mn ? 64u : (uint32_t)kBM};
+            ok = map_nd(&f.a, o.a_hi, 2, dims, str, box, o.a_stride);
+        }
         if (!ok) return fail(BRL_E_LAUNCH, "%s: cuTensorMapEncodeTiled failed", what);
         f.g = o.g;
         f.g.M = o.m_rows;
@@ -699,7 +901,7 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
         f.a_mn = o.a_mn;
         f.w_mn = o.w_mn;
         f.tile0 = tiles;
-        tiles += f.g.n_tiles;
+        tiles += K * f.g.n_tiles;
         f.dep = o.dep;
         f.dep_all = o.dep_all;
         if (o.dep >= 0) f.dep_count = 4u * (uint32_t)(o.dep_all ? fa.op[o.dep].g.n_tiles : fa.op[o.dep].g.n_tiles_n);
@@ -709,10 +911,17 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
     fa.nmb = nmb;
     fa.ready = ready;
     fa.trace = trace;
+    if constexpr (GROUPED) {
+        ga.K = K;
+        ga.sc_stride = grp->sc_stride;
+        ga.blob_stride = grp->blob_stride;
+        ga.grad_stride = grp->grad_stride;
+        ga.sumsq_stride = grp->sumsq_stride;
+    }
     static bool attr_set_dev[kMaxDevices] = {};
     bool& attr_set = attr_set_dev[device_slot()];
     if (!attr_set) {
-        if (cudaFuncSetAttribute(k_train_fused<kFBN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
+        if (cudaFuncSetAttribute(k_train_fused<kFBN, GROUPED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes) != cudaSuccess)
             return fail(BRL_E_LAUNCH, "%s: cannot reserve %u bytes of shared memory", what, Cfg::kSmemBytes);
         attr_set = true;
     }
@@ -727,7 +936,7 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
     at.val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = &at;
     cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, k_train_fused<kFBN>, fa) != cudaSuccess) return check_launch(what);
+    if (cudaLaunchKernelEx(&cfg, k_train_fused<kFBN, GROUPED>, ga) != cudaSuccess) return check_launch(what);
     return BRL_OK;
 }
 
@@ -735,10 +944,13 @@ static int32_t launch_fused_ops(cudaStream_t s, const OpSpec* ops, int n_ops, in
 
 using namespace brl;
 
+static int train_ops(OpSpec* fwd, OpSpec* bwd, unsigned char* sc, const unsigned char* blob, float* grads, double* grad_sumsq, int B);
+
 extern "C" {
 
 int64_t brl_mlp_num_params(void) { return (int64_t)flat_layout().total; }
 int64_t brl_mlp_train_blob_bytes(void) { return (int64_t)train_blob().total; }
+int64_t brl_mlp_param_stride(void) { return (int64_t)param_stride(); }
 int64_t brl_mlp_train_scratch_bytes(int64_t batch) { return batch > 0 ? (int64_t)train_scratch(batch).total : 0; }
 int64_t brl_mlp_train_trace_offset(int64_t batch) { return batch > 0 ? (int64_t)train_scratch(batch).trace : 0; }
 
@@ -850,37 +1062,174 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
     return launch_train_minibatch(s, t);
 }
 
+// ---- K learners, one optimizer step each, in the launches of one -------------------------------------------------------
+// scratch: K per-learner minibatch scratches (train_scratch(B), learner k's at k * total), then the grouped launches' tile
+// counters: [2 launches][kMaxOps][K][nmb + 1]
+static size_t grouped_ready_offset(int64_t K, int64_t B) { return (size_t)K * train_scratch(B).total; }
+static size_t grouped_ready_words(int64_t K, int64_t B) { return (size_t)2 * kMaxOps * K * (size_t)(ready_blocks(B) + 1); }
+
+int64_t brl_ppo_grad_grouped_scratch_bytes(int64_t n_learners, int64_t batch) {
+    if (n_learners <= 0 || batch <= 0 || n_learners > BRL_MAX_LEARNERS || batch > (1 << 24)) return 0;
+    return (int64_t)(grouped_ready_offset(n_learners, batch) + grouped_ready_words(n_learners, batch) * sizeof(uint32_t));
+}
+
+int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    if (opaque == nullptr || len != sizeof(BrlPpoGroupedParams))
+        return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: opaque must be one BrlPpoGroupedParams (%zu bytes), got %zu",
+                    sizeof(BrlPpoGroupedParams), len);
+    const BrlPpoGroupedParams* p = static_cast<const BrlPpoGroupedParams*>(opaque);
+    if (p->n_learners < 0 || p->n_learners > BRL_MAX_LEARNERS)
+        return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: n_learners must be in [0, %d]", BRL_MAX_LEARNERS);
+    if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: batch must be in [0, 2^24]");
+    if (p->n_learners == 0 || p->batch == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL
+    static const char* names[] = {"traj", "coefs", "blob", "scratch", "grads", "stats", "acc"};
+    for (int k = 0; k < 7; ++k)
+        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_ppo_grad_grouped: buffer '%s' is NULL", names[k]);
+    for (int k : {0, 2, 3, 4, 6})
+        if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_ppo_grad_grouped: buffer '%s' is not 16-byte aligned", names[k]);
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad_grouped: cuTensorMapEncodeTiled not available from the driver");
+    cudaStream_t s = (cudaStream_t)stream;
+    const char* what = "brl_ppo_grad_grouped";
+    const int K = p->n_learners, B = (int)p->batch;
+    const TrainScratch S = train_scratch(B);
+    const TrainBlob T = train_blob();
+    const FlatLayout F = flat_layout();
+    const long long* traj = static_cast<const long long*>(b[0]);
+    const float* coefs = static_cast<const float*>(b[1]);
+    const unsigned char* blob = static_cast<const unsigned char*>(b[2]);
+    unsigned char* sc = static_cast<unsigned char*>(b[3]);
+    float* grads = static_cast<float*>(b[4]);
+    float* stats = static_cast<float*>(b[5]);
+    unsigned char* acc = static_cast<unsigned char*>(b[6]);
+    double* grad_sumsq = reinterpret_cast<double*>(acc) + 14;  // learner k's |g|^2: f64 14 of its accumulator slice
+    const bool illegal_stat = (p->flags & BRL_PPO_ILLEGAL_STAT) != 0;
+    const int nmb = ready_blocks(B);
+    uint32_t* ready = reinterpret_cast<uint32_t*>(sc + grouped_ready_offset(K, B));
+    int32_t rc = BRL_OK;
+
+    // 0. tile counters and every learner's f64 accumulators
+    if (cudaMemsetAsync(ready, 0, grouped_ready_words(K, B) * sizeof(uint32_t), s) != cudaSuccess ||
+        cudaMemset2DAsync(acc, BRL_PPO_SCRATCH_BYTES, 0, 16 * sizeof(double), (size_t)K, s) != cudaSuccess)
+        return check_launch(what);
+    // 1. every learner's minibatch of observations
+    {
+        const dim3 grid((unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256), (unsigned)K);
+        uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
+        const long long st = (long long)S.total;
+        if (p->flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs_grouped<__nv_bfloat16>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
+        else if (p->flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs_grouped<uint8_t>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
+        else launch_pdl(k_gather_obs_grouped<float>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
+    }
+    // 2. the forward GEMMs of all learners as one launch, described by learner 0's ops: A operands (activations, dz) lie in
+    //    the scratch, B operands in the blob (forward, dgrad) or the scratch (wgrad)
+    OpSpec fwd[5], bwd[kMaxOps];
+    const int nb = train_ops(fwd, bwd, sc, blob, grads, grad_sumsq, B);
+    const GroupSpec grp{K, (long long)S.total, (long long)T.total, (long long)param_stride(), BRL_PPO_SCRATCH_BYTES / (long long)sizeof(double)};
+    for (OpSpec* o : {fwd + 0, fwd + 1, fwd + 2, fwd + 3, fwd + 4}) { o->a_stride = grp.sc_stride; o->w_stride = grp.blob_stride; }
+    for (int i = 0; i < nb; ++i) {
+        bwd[i].a_stride = grp.sc_stride;
+        bwd[i].w_stride = bwd[i].epi == kEpiWgrad ? grp.sc_stride : grp.blob_stride;
+    }
+    const int tune = p->reserved;
+    const bool wide_fwd = (tune & 4) != 0, wide_bwd = (tune & 16) == 0;  // the tile widths of launch_train_minibatch
+    rc = wide_fwd ? launch_fused_ops<128, true>(s, fwd, 5, nmb, ready, nullptr, what, &grp)
+                  : launch_fused_ops<64, true>(s, fwd, 5, nmb, ready, nullptr, what, &grp);
+    if (rc != BRL_OK) return rc;
+    if ((rc = check_launch(what)) != BRL_OK) return rc;
+    // 3. the loss heads
+    PpoGroupIO io{};
+    io.traj = traj;
+    io.coefs = coefs;
+    io.head.logits = reinterpret_cast<const float*>(sc + S.logits);
+    io.head.value = reinterpret_cast<const float*>(sc + S.value);
+    io.head.dlogits = reinterpret_cast<float*>(sc + S.dlogits);
+    io.head.dvalue = reinterpret_cast<float*>(sc + S.dvalue);
+    io.head.dz_hi = sc + S.dz5_hi;
+    io.head.dz_lo = sc + S.dz5_lo;
+    io.sc_stride = (long long)S.total;
+    io.stats = stats;
+    io.acc = acc;
+    io.batch = B;
+    io.K = K;
+    io.flags = p->flags & (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
+    if ((rc = launch_ppo_loss_grouped(s, io)) != BRL_OK) return rc;
+    // 4. the backward GEMMs
+    uint32_t* ready_bwd = ready + (size_t)kMaxOps * K * (nmb + 1);
+    rc = wide_bwd ? launch_fused_ops<128, true>(s, bwd, nb, nmb, ready_bwd, nullptr, what, &grp)
+                  : launch_fused_ops<64, true>(s, bwd, nb, nmb, ready_bwd, nullptr, what, &grp);
+    if (rc != BRL_OK) return rc;
+    // 5. bias gradients (and the deferred illegal-action statistics)
+    {
+        GroupedBiasArgs g{};
+        for (int l = 0; l < 4; ++l) {
+            g.a.hi[l] = reinterpret_cast<const __nv_bfloat16*>(sc + S.dz_hi[l]);
+            g.a.lo[l] = reinterpret_cast<const __nv_bfloat16*>(sc + S.dz_lo[l]);
+        }
+        g.a.dlogits = io.head.dlogits;
+        g.a.dvalue = io.head.dvalue;
+        g.a.grads = grads;
+        g.a.B = B;
+        g.a.F = F;
+        g.traj = traj;
+        g.coefs = coefs;
+        g.logits = io.head.logits;
+        g.stats = stats;
+        g.acc = acc;
+        g.sc_stride = (long long)S.total;
+        g.illegal_stat = illegal_stat;
+        g.n_gram = gram_blocks(B, 1024);
+        launch_pdl(k_bias_grad_grouped, dim3(4 * (kHidden / 64) + 1 + (illegal_stat ? 1 : 0), (unsigned)K), dim3(1024), 0, s, g);
+    }
+    return check_launch(what);
+}
+
+int32_t brl_mlp_adam_step_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    if ((opaque == nullptr && len != 0) || len % sizeof(BrlAdamParams) != 0)
+        return fail(BRL_E_OPAQUE, "brl_mlp_adam_step_grouped: opaque must be an array of BrlAdamParams (%zu bytes each), got %zu bytes",
+                    sizeof(BrlAdamParams), len);
+    const int64_t K = (int64_t)(len / sizeof(BrlAdamParams));
+    if (K == 0) return BRL_OK;  // no learners: a no-op, its buffers may be NULL
+    if (K > BRL_MAX_LEARNERS) return fail(BRL_E_OPAQUE, "brl_mlp_adam_step_grouped: at most %d learners", BRL_MAX_LEARNERS);
+    static const char* names[] = {"params", "grads", "m", "v", "acc", "blob"};
+    for (int k = 0; k < 6; ++k) {
+        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_mlp_adam_step_grouped: buffer '%s' is NULL", names[k]);
+        if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_mlp_adam_step_grouped: buffer '%s' is not 16-byte aligned", names[k]);
+    }
+    const BrlAdamParams* p = static_cast<const BrlAdamParams*>(opaque);
+    GroupedAdamArgs g{};
+    for (int64_t k = 0; k < K; ++k) {
+        if (p[k].n != (int64_t)flat_layout().total || p[k].step <= 0)
+            return fail(BRL_E_OPAQUE, "brl_mlp_adam_step_grouped: learner %lld: n must be brl_mlp_num_params() and step (1-based) > 0", (long long)k);
+        AdamLearner& l = g.l[k];
+        l.max_norm = p[k].max_grad_norm; l.lr = p[k].lr; l.b1 = p[k].beta1; l.b2 = p[k].beta2; l.eps = p[k].eps;
+        l.bc1 = 1.0f - powf(p[k].beta1, (float)p[k].step);  // as brl_mlp_adam_step
+        l.bc2 = 1.0f - powf(p[k].beta2, (float)p[k].step);
+    }
+    g.a.p = static_cast<float*>(b[0]);
+    g.a.g = static_cast<const float*>(b[1]);
+    g.a.m = static_cast<float*>(b[2]);
+    g.a.v = static_cast<float*>(b[3]);
+    g.a.sumsq = static_cast<const double*>(b[4]) + 14;
+    g.a.blob = static_cast<unsigned char*>(b[5]);
+    g.a.F = flat_layout();
+    g.a.T = train_blob();
+    g.sumsq_stride = BRL_PPO_SCRATCH_BYTES / (long long)sizeof(double);
+    launch_pdl(k_adam_pack_grouped, dim3(adam_pack_grid(), (unsigned)K), dim3(256), 0, (cudaStream_t)stream, g);
+    return check_launch("brl_mlp_adam_step_grouped");
+}
+
 }  // extern "C"
 
-int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
-    const int B = (int)t.batch;
+// The GEMMs of one minibatch: fwd[5] and bwd[] (returns the number of backward ops)
+static int train_ops(OpSpec* fwd, OpSpec* bwd, unsigned char* sc, const unsigned char* blob, float* grads, double* grad_sumsq, int B) {
     const TrainBlob T = train_blob();
     const FlatLayout F = flat_layout();
     const TrainScratch S = train_scratch(B);
-    const unsigned char* blob = t.blob;
-    unsigned char* sc = t.scratch;
-    float* grads = t.grads;
     auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(sc + off); };
-    int32_t rc = BRL_OK;
-
-    // 0. counters and accumulators first, so that nothing but kernels (launched with programmatic dependent launch) follows
-    if (cudaMemsetAsync(sc + S.ready, 0, ready_words(B) * sizeof(uint32_t), s) != cudaSuccess ||
-        (t.zero != nullptr && cudaMemsetAsync(t.zero, 0, t.zero_bytes, s) != cudaSuccess))
-        return check_launch(t.what);
-    // 1. minibatch gather of the observation (src/update.py:194-199, cast of src/update.py:95)
-    {
-        const unsigned grid = (unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256);
-        uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
-        if (t.obs_flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs<__nv_bfloat16>, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(t.obs), t.index, (int64_t)B, o);
-        else if (t.obs_flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs<uint8_t>, dim3(grid), dim3(256), 0, s, static_cast<const uint8_t*>(t.obs), t.index, (int64_t)B, o);
-        else launch_pdl(k_gather_obs<float>, dim3(grid), dim3(256), 0, s, static_cast<const float*>(t.obs), t.index, (int64_t)B, o);
-    }
     // 2. the GEMMs.  Forward: layers 1..4 (activations kept, row-major bf16 hi / lo: next layer's A, the ReLU mask, the
     //    wgrad's MN-major A) + the head.  Backward: dgrad into layer l's pre-activation, dz_l = (dz_{l+1} . W_{l+1}^T) * [h_l > 0]
     //    (S.dz_*[l-1], l = 1..4), and the wgrads dW_l = h_{l-1}^T . dz_l straight from the row-major h and dz.
-    // |grads|^2 accumulates in t.grad_sumsq (cleared by the caller before the loss head, which runs before every wgrad)
-    double* grad_sumsq = t.grad_sumsq;
-    OpSpec fwd[5], bwd[kMaxOps];
+    // |grads|^2 accumulates in grad_sumsq (cleared by the caller before the loss head, which runs before every wgrad)
     for (int l = 0; l < 5; ++l) {  // forward: A = previous activation (K-major), W = Wn[l] [in, out_pad] (MN-major)
         OpSpec& o = fwd[l];
         o = OpSpec{};
@@ -953,6 +1302,33 @@ int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
         add_wgrad(2);
         add_wgrad(1);
     }
+    return nb;
+}
+
+int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
+    const int B = (int)t.batch;
+    const FlatLayout F = flat_layout();
+    const TrainScratch S = train_scratch(B);
+    unsigned char* sc = t.scratch;
+    float* grads = t.grads;
+    auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(sc + off); };
+    int32_t rc = BRL_OK;
+
+    // 0. counters and accumulators first, so that nothing but kernels (launched with programmatic dependent launch) follows
+    if (cudaMemsetAsync(sc + S.ready, 0, ready_words(B) * sizeof(uint32_t), s) != cudaSuccess ||
+        (t.zero != nullptr && cudaMemsetAsync(t.zero, 0, t.zero_bytes, s) != cudaSuccess))
+        return check_launch(t.what);
+    // 1. minibatch gather of the observation (src/update.py:194-199, cast of src/update.py:95)
+    {
+        const unsigned grid = (unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256);
+        uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
+        if (t.obs_flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs<__nv_bfloat16>, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(t.obs), t.index, (int64_t)B, o);
+        else if (t.obs_flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs<uint8_t>, dim3(grid), dim3(256), 0, s, static_cast<const uint8_t*>(t.obs), t.index, (int64_t)B, o);
+        else launch_pdl(k_gather_obs<float>, dim3(grid), dim3(256), 0, s, static_cast<const float*>(t.obs), t.index, (int64_t)B, o);
+    }
+    OpSpec fwd[5], bwd[kMaxOps];
+    const int nb = train_ops(fwd, bwd, sc, t.blob, grads, t.grad_sumsq, B);
+    double* grad_sumsq = t.grad_sumsq;
     const int nmb = ready_blocks(B);
     uint32_t* ready = reinterpret_cast<uint32_t*>(sc + S.ready);
     unsigned long long* trace = (t.tune & 8) ? reinterpret_cast<unsigned long long*>(sc + S.trace) : nullptr;  // tune bit 3

@@ -43,6 +43,7 @@ struct PpoArgs {
 // acc slots
 enum { kAccAdv = 0, kAccAdv2, kAccIll, kAccActor, kAccValue, kAccEnt, kAccKl, kAccClip, kAccGramTicket = 13, kAccTicket = 15 };
 static_assert(128 + 40 * 8 <= 512 && 512 + kGramBlocks * kGramN * 4 <= BRL_PPO_SCRATCH_BYTES, "scratch layout");
+static_assert(kAccGramTicket == 13, "gram_args_at (ppo_gram.cuh) places the Gram ticket in f64 13");
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -81,8 +82,54 @@ struct Row {
     }
 };
 
+// ---- the loss head of K learners at once (brl_ppo_grad_grouped): blockIdx.y = learner --------------------------------
+// `a` holds learner 0's scratch pointers and the shared flags; learner k's trajectory comes from row k of the device
+// table, its coefficients from row k of `coefs`, and its minibatch scratch / accumulators lie k strides further.
+struct PpoGroupArgs {
+    PpoArgs a;
+    const long long* traj;   // [K][8]: obs, index, mask, action, old_log_prob, old_value, advantages, targets
+    const float* coefs;      // [K][4]: clip_eps, ent_coef, vf_coef, illegal_l2_coef
+    long long sc_stride;     // bytes between learners' minibatch scratch (logits, value, dlogits, dvalue, dz)
+    long long acc_stride;    // bytes between learners' accumulator scratch
+    int illegal_stat;        // BRL_PPO_ILLEGAL_STAT
+};
+__device__ __forceinline__ PpoArgs learner_ppo_args(const PpoGroupArgs& g, int k) {
+    PpoArgs a = g.a;
+    auto sc = [&](auto* p) { return (decltype(p))((const char*)p + k * g.sc_stride); };
+    const long long* t = g.traj + 8 * k;
+    a.logits = sc(a.logits);
+    a.value = sc(a.value);
+    a.dlogits = sc(a.dlogits);
+    a.dvalue = sc(a.dvalue);
+    a.dz_hi = sc(a.dz_hi);
+    a.dz_lo = sc(a.dz_lo);
+    a.index = reinterpret_cast<const int32_t*>(t[1]);
+    a.mask = reinterpret_cast<const uint8_t*>(t[2]);
+    a.action = reinterpret_cast<const int32_t*>(t[3]);
+    a.old_log_prob = reinterpret_cast<const float*>(t[4]);
+    a.old_value = reinterpret_cast<const float*>(t[5]);
+    a.adv = reinterpret_cast<const float*>(t[6]);
+    a.targets = reinterpret_cast<const float*>(t[7]);
+    a.stats += 8 * k;
+    a.acc = reinterpret_cast<double*>(reinterpret_cast<char*>(a.acc) + k * g.acc_stride);
+    a.spec = reinterpret_cast<double*>(reinterpret_cast<char*>(a.acc) + 128);
+    a.gram_part = reinterpret_cast<float*>(reinterpret_cast<char*>(a.acc) + 512);
+    a.clip_eps = g.coefs[4 * k];
+    a.ent_coef = g.coefs[4 * k + 1];
+    a.vf_coef = g.coefs[4 * k + 2];
+    a.ill_coef = g.coefs[4 * k + 3];
+    // as brl_ppo_grad: with a zero coefficient the norm is only a statistic, formed (if asked for) beside the bias sums
+    a.defer_illegal = a.ill_coef == 0.0f;
+    a.skip_illegal = a.defer_illegal && !g.illegal_stat;
+    return a;
+}
+__device__ __forceinline__ const PpoArgs& learner_args(const PpoArgs& a) { return a; }
+__device__ __forceinline__ PpoArgs learner_args(const PpoGroupArgs& g) { return learner_ppo_args(g, blockIdx.y); }
+
 // sum over the minibatch of advantages and advantages^2 (reward scaling, src/update.py:35-36)
-__global__ void __launch_bounds__(128) k_ppo_prepass(const PpoArgs a) {
+template <class Args>  // PpoArgs, or PpoGroupArgs (blockIdx.y = learner)
+__global__ void __launch_bounds__(128) k_ppo_prepass(const Args g) {
+    const PpoArgs& a = learner_args(g);
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
     double s_adv = 0.0, s_adv2 = 0.0;
@@ -142,9 +189,11 @@ __device__ __forceinline__ void ppo_finalize(const PpoArgs& a) {
     a.stats[7] = 0.0f;
 }
 
-__global__ void __launch_bounds__(128) k_ppo_loss(const PpoArgs a, int have_prepass) {
+template <class Args>  // PpoArgs, or PpoGroupArgs (blockIdx.y = learner)
+__global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass) {
     pdl_trigger();
     pdl_wait();
+    const PpoArgs& a = learner_args(g);
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
     const float invB = 1.0f / (float)a.B;
@@ -260,6 +309,19 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const PpoArgs a, int have_prep
     }
 }
 
+// a learner with a non-zero coefficient forms its norm here in full (partials + tail: the loss gradient needs v_1), one
+// with the statistic asked for only the partials, the others nothing
+__global__ void __launch_bounds__(1024) k_ppo_gram_grouped(const PpoGroupArgs g) {
+    __shared__ GramSmem sm;
+    pdl_trigger();
+    pdl_wait();
+    const PpoArgs a = learner_ppo_args(g, blockIdx.y);
+    if (a.skip_illegal) return;
+    const GramArgs ga = gram_args_at(a.logits, a.index, a.mask, a.B, reinterpret_cast<unsigned char*>(a.acc), nullptr);
+    if (a.defer_illegal) gram_partial<1024>(ga, (int)blockIdx.x, (int)gridDim.x, sm.X);
+    else gram_block<1024>(ga, (int)blockIdx.x, (int)gridDim.x, sm);
+}
+
 
 // ---- optimizer: optax.chain(clip_by_global_norm(c), adam(lr, eps=1e-5)) (ppo.py:195-211) -------
 // VEC = 4: 128-bit accesses over the first n / 4 * 4 elements (16-byte-aligned buffers), the <= 3 tail elements by block 0
@@ -366,17 +428,8 @@ int brl::gram_blocks(int64_t B, int threads) {
 }
 
 brl::GramArgs brl::gram_args(void** b, const BrlPpoParams* p, float* stat) {
-    GramArgs g{};
-    g.logits = static_cast<const float*>(b[0]);
-    g.index = static_cast<const int32_t*>(b[2]);
-    g.mask = static_cast<const uint8_t*>(b[3]);
-    g.B = p->batch;
-    g.ticket = reinterpret_cast<unsigned long long*>(static_cast<double*>(b[12]) + kAccGramTicket);
-    g.spec = reinterpret_cast<double*>(static_cast<unsigned char*>(b[12]) + 128);
-    g.part = reinterpret_cast<float*>(static_cast<unsigned char*>(b[12]) + 512);
-    g.stat = stat;
-    g.tol = stat ? 3e-4f : 1e-6f;  // statistic only (deferred) vs v_1 feeding the loss gradient
-    return g;
+    return gram_args_at(static_cast<const float*>(b[0]), static_cast<const int32_t*>(b[2]), static_cast<const uint8_t*>(b[3]),
+                        p->batch, static_cast<unsigned char*>(b[12]), stat);
 }
 
 int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* p, void* dz_hi, void* dz_lo, bool acc_zeroed,
@@ -418,7 +471,7 @@ int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* 
     unsigned grid = (unsigned)((a.B + 3) / 4);
     if (grid > 148u * 8u) grid = 148u * 8u;
     const int prepass = a.reward_scaling;
-    if (prepass) k_ppo_prepass<<<grid > 32u ? 32u : grid, 128, 0, s>>>(a);
+    if (prepass) k_ppo_prepass<PpoArgs><<<grid > 32u ? 32u : grid, 128, 0, s>>>(a);
     a.defer_illegal = defer_illegal && a.ill_coef == 0.0f;
     a.skip_illegal = a.defer_illegal && !(p->flags & BRL_PPO_ILLEGAL_STAT);
     if (!a.skip_illegal) {
@@ -428,7 +481,7 @@ int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* 
         if (prepass) kern<<<gram_blocks, 1024, 0, s>>>(g);  // a plain launch may not be followed by a PDL one that skips it
         else launch_pdl(kern, dim3(gram_blocks), dim3(1024), 0, s, g);
     }
-    launch_pdl(k_ppo_loss, dim3(grid), dim3(128), 0, s, a, prepass);
+    launch_pdl(k_ppo_loss<PpoArgs>, dim3(grid), dim3(128), 0, s, a, prepass);
     return check_launch("brl_ppo_loss");
 }
 
@@ -497,3 +550,36 @@ int32_t brl_gather_rows(brl_stream_t stream, void** b, const void* opaque, size_
 }
 
 }  // extern "C"
+
+int32_t brl::launch_ppo_loss_grouped(cudaStream_t s, const PpoGroupIO& io) {
+    PpoGroupArgs g{};
+    PpoArgs& a = g.a;
+    a.logits = io.head.logits;
+    a.value = io.head.value;
+    a.dlogits = io.head.dlogits;
+    a.dvalue = io.head.dvalue;
+    a.dz_hi = static_cast<unsigned short*>(io.head.dz_hi);
+    a.dz_lo = static_cast<unsigned short*>(io.head.dz_lo);
+    a.stats = io.stats;
+    a.acc = reinterpret_cast<double*>(io.acc);
+    a.B = io.batch;
+    a.value_clipping = (io.flags & BRL_PPO_VALUE_CLIPPING) != 0;
+    a.reward_scaling = (io.flags & BRL_PPO_REWARD_SCALING) != 0;
+    a.masked_policy = (io.flags & BRL_PPO_UNMASKED_POLICY) == 0;
+    g.traj = io.traj;
+    g.coefs = io.coefs;
+    g.sc_stride = io.sc_stride;
+    g.acc_stride = BRL_PPO_SCRATCH_BYTES;
+    g.illegal_stat = (io.flags & BRL_PPO_ILLEGAL_STAT) != 0;
+    const unsigned K = (unsigned)io.K;
+    // the grids of launch_ppo_loss, one row per learner
+    unsigned grid = (unsigned)((a.B + 3) / 4);
+    if (grid > 148u * 8u) grid = 148u * 8u;
+    const int prepass = a.reward_scaling;
+    if (prepass) k_ppo_prepass<PpoGroupArgs><<<dim3(grid > 32u ? 32u : grid, K), 128, 0, s>>>(g);
+    const dim3 gram_grid((unsigned)brl::gram_blocks(a.B, 1024), K);
+    if (prepass) k_ppo_gram_grouped<<<gram_grid, 1024, 0, s>>>(g);  // a plain launch may not be followed by a PDL one that skips it
+    else launch_pdl(k_ppo_gram_grouped, gram_grid, dim3(1024), 0, s, g);
+    launch_pdl(k_ppo_loss<PpoGroupArgs>, dim3(grid, K), dim3(128), 0, s, g, prepass);
+    return check_launch("brl_ppo_grad_grouped");
+}

@@ -114,6 +114,23 @@ struct TrainMinibatch {
 };
 int32_t launch_train_minibatch(cudaStream_t stream, const TrainMinibatch& t);
 
+// brl_ppo_grad_grouped's loss head (brl_ppo.cu): launch_ppo_loss for K learners, one grid row per learner.  Learner k's
+// trajectory buffers are row k of the device table `traj`, its coefficients row k of `coefs`; its forward outputs and
+// d loss buffers lie k * sc_stride bytes after learner 0's `head`, its stats at stats + 8k, its f64 accumulators (cleared
+// by the caller) at acc + k * BRL_PPO_SCRATCH_BYTES.  A zero illegal_l2_coef defers the logged statistic to the bias sums.
+struct PpoGroupIO {
+    const long long* traj;  // [K][8]: obs, index, mask, action, old_log_prob, old_value, advantages, targets
+    const float* coefs;     // [K][4]: clip_eps, ent_coef, vf_coef, illegal_l2_coef
+    TrainHeadIO head;
+    long long sc_stride;
+    float* stats;
+    unsigned char* acc;
+    int64_t batch;
+    int K;
+    int32_t flags;
+};
+int32_t launch_ppo_loss_grouped(cudaStream_t stream, const PpoGroupIO& io);
+
 // Programmatic dependent launch for the short kernels of a dependent chain (the PPO optimizer step): the kernel may be
 // scheduled while its predecessor in the stream drains; it must execute pdl_wait() before touching global memory and
 // should call pdl_trigger() first so that ITS successor can be scheduled early too.

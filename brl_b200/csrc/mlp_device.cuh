@@ -72,6 +72,11 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map
         "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
         ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
+__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2, int c3, int c4) {
+    asm volatile(
+        "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
+        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4) : "memory");
+}
 // shared -> global tile store through the TMA (bulk async-group completion)
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t src, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
@@ -209,10 +214,10 @@ static bool make_map_store(CUtensorMap* m, const void* ptr, uint64_t rows, uint6
                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// general bf16 tensor map (rank <= 4), 128B swizzle, zero fill: dims / box innermost first, strides in bytes for dims 1..
+// general bf16 tensor map (rank <= 5), 128B swizzle, zero fill: dims / box innermost first, strides in bytes for dims 1..
 static inline bool make_map_nd(CUtensorMap* m, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box) {
-    cuuint64_t d[4], s[3];
-    cuuint32_t b[4], e[4] = {1, 1, 1, 1};
+    cuuint64_t d[5], s[4];
+    cuuint32_t b[5], e[5] = {1, 1, 1, 1, 1};
     for (int i = 0; i < rank; ++i) { d[i] = dims[i]; b[i] = box[i]; }
     for (int i = 0; i + 1 < rank; ++i) s[i] = strides_bytes[i];
     return encode_fn()(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(ptr), d, s, b, e, CU_TENSOR_MAP_INTERLEAVE_NONE,

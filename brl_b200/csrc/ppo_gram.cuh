@@ -37,6 +37,23 @@ struct GramArgs {
     float tol;              // power iteration stops when no component of v moved by more than this over 8 steps
 };
 
+// GramArgs of one minibatch whose f64 accumulators are `acc` (BRL_PPO_SCRATCH_BYTES: the ticket is f64 13, the spectrum
+// starts at byte 128, the partials at byte 512); stat != NULL: the statistic alone is wanted
+__host__ __device__ inline GramArgs gram_args_at(const float* logits, const int32_t* index, const uint8_t* mask, int64_t B,
+                                                 unsigned char* acc, float* stat) {
+    GramArgs g{};
+    g.logits = logits;
+    g.index = index;
+    g.mask = mask;
+    g.B = B;
+    g.ticket = reinterpret_cast<unsigned long long*>(acc + 13 * sizeof(double));
+    g.spec = reinterpret_cast<double*>(acc + 128);
+    g.part = reinterpret_cast<float*>(acc + 512);
+    g.stat = stat;
+    g.tol = stat ? 3e-4f : 1e-6f;  // statistic only (deferred) vs v_1 feeding the loss gradient
+    return g;
+}
+
 struct GramSmem {
     float X[64 * kGramPad];        // staging of 64 sample rows (gram_partial<1024>)
     double Gd[kGramN];             // G in double (final Rayleigh quotient)

@@ -76,6 +76,8 @@
     X(brl_match_stats_ranges, "iix") \
     X(brl_duplicate_match, "iiiiisoxooooooooooooo") \
     X(brl_evaluate_match, "iiisooxooooooooooooooooooo") \
+    X(brl_ppo_grad_grouped, "iiisoos") \
+    X(brl_mlp_adam_step_grouped, "xixxix") \
     /* end */
 
 namespace {

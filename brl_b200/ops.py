@@ -415,6 +415,85 @@ def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, a
                            _ptr(old_value), _ptr(adv), _ptr(targets), _ptr(grads), _ptr(stats), _ptr(acc)], p)
 
 
+# ---- population training: K learners' optimizer steps in the launches of one (brl_ppo_grad_grouped) ----------------------
+def ppo_grad_grouped_scratch_bytes(n_learners: int, batch: int) -> int:
+    return _size_query("brl_ppo_grad_grouped_scratch_bytes", n_learners, batch)
+
+
+def mlp_param_stride() -> int:
+    """floats between two learners' rows of a population's [K, stride] parameter / gradient / moment buffers (a learner
+    uses the first mlp_num_params() of its row)"""
+    return _size_query("brl_mlp_param_stride")
+
+
+def ppo_trajectory_row(obs, index, mask, action, old_log_prob, old_value, adv, targets) -> list:
+    """One learner's row of the trajectory table of `ppo_grad_grouped`: the device addresses of its `ppo_grad` buffers
+    (index may be None = identity).  The tensors must stay alive while a call that reads the table is in flight."""
+    if obs.dtype == torch.bool:
+        obs = obs.view(torch.uint8)
+    return [_ptr(obs), _ptr(index) or 0, _ptr(mask), _ptr(action), _ptr(old_log_prob), _ptr(old_value), _ptr(adv), _ptr(targets)]
+
+
+def ppo_grad_grouped(traj, coefs, blob, scratch, grads, stats, acc, *, batch: int, obs_dtype, value_clipping=True,
+                     reward_scaling=False, masked_policy=True, illegal_stat: bool = True, tune: int = 0) -> None:
+    """`ppo_grad` for K learners in one set of launches.  traj: CUDA int64[K, 8] rows of `ppo_trajectory_row`; coefs: CUDA
+    float32[K, 4] = (clip_eps, ent_coef, vf_coef, illegal_l2_coef) per learner; blob: uint8[K, mlp_train_blob_bytes];
+    grads: float32[K, mlp_param_stride]; stats: float32[K, 8]; acc: float64[K, PPO_SCRATCH_BYTES / 8], whose row k holds
+    learner k's |grads|^2 at element 14 on return.  Every learner's minibatch has `batch` rows and observations of
+    `obs_dtype`; learner k's results are bit-identical to `ppo_grad` with its own buffers and coefficients."""
+    L = _lib.load()
+    K = int(traj.shape[0]) if traj.dim() == 2 else -1
+    if traj.dtype != torch.int64 or traj.dim() != 2 or traj.shape[1] != 8:
+        raise _lib.BrlError("ppo_grad_grouped: traj must be int64[K, 8] (ops.ppo_trajectory_row)")
+    if K > _lib.MAX_LEARNERS:
+        raise _lib.BrlError(f"ppo_grad_grouped: at most {_lib.MAX_LEARNERS} learners")
+    if coefs.dtype != torch.float32 or tuple(coefs.shape) != (K, 4):
+        raise _lib.BrlError("ppo_grad_grouped: coefs must be float32[K, 4]")
+    n, nb = mlp_param_stride(), L.brl_mlp_train_blob_bytes()
+    if grads.dtype != torch.float32 or grads.numel() != K * n or stats.dtype != torch.float32 or stats.numel() != K * 8:
+        raise _lib.BrlError("ppo_grad_grouped: grads must be float32[K, mlp_param_stride], stats float32[K, 8]")
+    if blob.numel() != K * nb or scratch.numel() < ppo_grad_grouped_scratch_bytes(K, batch) or \
+            acc.dtype != torch.float64 or acc.numel() != K * (_lib.PPO_SCRATCH_BYTES // 8):
+        raise _lib.BrlError("ppo_grad_grouped: blob must be uint8[K, mlp_train_blob_bytes], acc float64[K, PPO_SCRATCH_BYTES / 8], "
+                            "scratch ppo_grad_grouped_scratch_bytes(K, batch)")
+    try:
+        oflag = {torch.float32: 0, torch.uint8: _lib.PPO_OBS_U8, torch.bool: _lib.PPO_OBS_U8,
+                 torch.bfloat16: _lib.PPO_OBS_BF16}[obs_dtype]
+    except KeyError:
+        raise _lib.BrlError(f"ppo_grad_grouped: observation dtype {obs_dtype} not supported") from None
+    flags = (_lib.PPO_VALUE_CLIPPING if value_clipping else 0) | (_lib.PPO_REWARD_SCALING if reward_scaling else 0) | \
+            (0 if masked_policy else _lib.PPO_UNMASKED_POLICY) | (_lib.PPO_ILLEGAL_STAT if illegal_stat else 0) | oflag
+    p = _lib.BrlPpoGroupedParams(int(batch), K, flags, int(tune), 0)
+    _call("brl_ppo_grad_grouped", [_ptr(traj), _ptr(coefs), _ptr(blob), _ptr(scratch), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+
+
+def mlp_adam_step_grouped(params, grads, m, v, acc, blob, *, steps, lrs, max_grad_norms, beta1=0.9, beta2=0.999,
+                          eps=1e-5) -> None:
+    """`mlp_adam_step` for K learners in one launch: params / grads / m / v float32[K, mlp_param_stride], blob
+    uint8[K, mlp_train_blob_bytes], acc = `ppo_grad_grouped`'s float64[K, PPO_SCRATCH_BYTES / 8].  steps, lrs,
+    max_grad_norms (and beta1, beta2, eps when given as sequences): one entry per learner."""
+    L = _lib.load()
+    K = len(steps)
+    if len(lrs) != K or len(max_grad_norms) != K:
+        raise _lib.BrlError("mlp_adam_step_grouped: steps, lrs and max_grad_norms need one entry per learner")
+    if K > _lib.MAX_LEARNERS:
+        raise _lib.BrlError(f"mlp_adam_step_grouped: at most {_lib.MAX_LEARNERS} learners")
+    n, stride = L.brl_mlp_num_params(), mlp_param_stride()
+    for name, t in (("params", params), ("grads", grads), ("m", m), ("v", v)):
+        if t.dtype != torch.float32 or t.numel() != K * stride:
+            raise _lib.BrlError(f"mlp_adam_step_grouped: {name} must be float32[K, mlp_param_stride]")
+    if acc.dtype != torch.float64 or acc.numel() != K * (_lib.PPO_SCRATCH_BYTES // 8) or \
+            blob.numel() != K * L.brl_mlp_train_blob_bytes():
+        raise _lib.BrlError("mlp_adam_step_grouped: acc must be float64[K, PPO_SCRATCH_BYTES / 8], blob uint8[K, mlp_train_blob_bytes]")
+
+    def per(x):
+        return list(x) if isinstance(x, (list, tuple)) else [x] * K
+    b1, b2, ep = per(beta1), per(beta2), per(eps)
+    p = (_lib.BrlAdamParams * K)(*[_lib.BrlAdamParams(n, int(steps[k]), float(lrs[k]), float(b1[k]), float(b2[k]), float(ep[k]),
+                                                       float(max_grad_norms[k])) for k in range(K)])
+    _call("brl_mlp_adam_step_grouped", [_ptr(params), _ptr(grads), _ptr(m), _ptr(v), _ptr(acc), _ptr(blob)], p)
+
+
 def sl_examples(table, calls, offsets, traj, obs, mask, label, *, position=None, position_out=None, seed=0, step=0,
                 env_offset=0) -> None:
     """make_dataset of sl.py:100-117 for a batch: example b replays trajectory traj[b] up to its call `position[b]` (drawn

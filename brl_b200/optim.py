@@ -11,11 +11,12 @@ from . import ops
 from .models import LAYERS
 
 
-def flatten_params(params, clone: bool = True):
-    """-> (flat fp32 buffer, params dict whose tensors are views into it, in LAYERS order w then b)."""
+def flatten_params(params, clone: bool = True, out: Optional[torch.Tensor] = None):
+    """-> (flat fp32 buffer, params dict whose tensors are views into it, in LAYERS order w then b).  `out`: the flat
+    buffer to fill (e.g. one learner's row of a stacked population buffer) instead of a new one."""
     tensors = [params[name][k] for name in LAYERS for k in ("w", "b")]
     n = sum(t.numel() for t in tensors)
-    flat = torch.empty(n, dtype=torch.float32, device=tensors[0].device)
+    flat = torch.empty(n, dtype=torch.float32, device=tensors[0].device) if out is None else out
     out, off = {}, 0
     for name in LAYERS:
         out[name] = {}
@@ -68,6 +69,18 @@ class AdamWithClip:
         ops.mlp_adam_step(flat_params, flat_grads, state.mu, state.nu, sumsq, blob, step=state.count + 1, lr=self.lr_at(state.count),
                           beta1=self.b1, beta2=self.b2, eps=self.eps, max_grad_norm=self.max_grad_norm)
         return OptState(state.count + 1, state.mu, state.nu)
+
+
+def update_mlp_grouped_(optimizers, flat_params, flat_grads, m, v, states, acc, blob):
+    """`AdamWithClip.update_mlp_` for K learners in one launch (ops.mlp_adam_step_grouped): flat_params / flat_grads / m /
+    v float32[K, ops.mlp_param_stride()] with states[k].mu / .nu = m[k, :n] / v[k, :n], acc the float64[K, ...] scratch of `ops.ppo_grad_grouped`, blob
+    uint8[K, ...].  Each learner steps with its own optimizer's learning rate (schedule), clipping, betas and eps.
+    Returns the advanced states."""
+    ops.mlp_adam_step_grouped(flat_params, flat_grads, m, v, acc, blob, steps=[st.count + 1 for st in states],
+                              lrs=[o.lr_at(st.count) for o, st in zip(optimizers, states)],
+                              max_grad_norms=[o.max_grad_norm for o in optimizers], beta1=[o.b1 for o in optimizers],
+                              beta2=[o.b2 for o in optimizers], eps=[o.eps for o in optimizers])
+    return [OptState(st.count + 1, st.mu, st.nu) for st in states]
 
 
 def make_optimizer(config) -> AdamWithClip:

@@ -28,7 +28,7 @@ from .gae import make_calc_gae
 from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
 from .optim import make_optimizer
 from .roll_out import make_roll_out
-from .update import make_update_step
+from .update import check_population_configs, make_population_update_step, make_update_step
 from .zoo import ModelZoo, device_zoo_fits
 
 
@@ -79,173 +79,247 @@ def make_evaluators(config: dict, eval_env, eval_opp_params):
                                  duplicate=True, team2_params=eval_opp_params))
 
 
+def full_config(config: dict) -> dict:
+    """default_config() updated with `config`, and the derived num_updates / num_minibatches"""
+    cfg = dict(default_config())
+    cfg.update(config)
+    cfg["num_updates"] = cfg["total_timesteps"] // cfg["num_steps"] // cfg["num_envs"]   # ppo.py:225-227
+    cfg["num_minibatches"] = cfg["num_envs"] * cfg["num_steps"] // cfg["minibatch_size"]  # ppo.py:228-230
+    return cfg
+
+
+class Learner:
+    """One run's control plane of `train`: set-up, and per iteration the evaluations, opponent / zoo choice, rollout and
+    GAE (`collect`), then logging and table rotation (`finish_iteration`) around an update step the caller runs -- alone
+    (`train`) or grouped with other learners' (`train_population`)."""
+
+    def __init__(self, config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=None, device="cuda",
+                 log_fn: Optional[Callable[[dict], None]] = None, eval_opp_params=None,
+                 np_rng: Optional[np.random.Generator] = None, forward_pass_factory=None):
+        make_fp = forward_pass_factory or make_forward_pass
+        self.config = config = full_config(config)
+        self.log_fn = log_fn
+        self.np_rng = np_rng or np.random.default_rng(config["seed"])
+        self.dev = dev = torch.device(device)
+
+        def as_table(t):
+            return _deals.load_table(t) if isinstance(t, str) else np.asarray(t, dtype=np.uint8)
+
+        if tables is None:
+            d = config["dds_results_dir"]
+            if os.path.isdir(d):
+                tables = [os.path.join(d, f) for f in sorted(os.listdir(d)) if "train" in f]            # ppo.py:292-294
+                if eval_table is None and os.path.exists(os.path.join(d, "test_000.npy")):
+                    eval_table = os.path.join(d, "test_000.npy")                                      # ppo.py:252
+            else:
+                tables = [_deals.synthetic_deal_table(config["hash_size"], seed=config["seed"] + k) for k in range(2)]
+        tables = [as_table(t) for t in tables]
+        eval_table = as_table(eval_table) if eval_table is not None else _deals.synthetic_deal_table(config["hash_size"], seed=10_000)
+
+        self.optimizer = make_optimizer(config)                                                       # ppo.py:195-211
+        self.actor_forward_pass = make_fp(config["actor_activation"], config["actor_model_type"])
+        rng, _rng = brandom.split(rng)
+        params = init_params(_rng & 0x7FFFFFFF, dev)                                                  # ppo.py:240-243
+        opt_state = self.optimizer.init(params)
+        if config["load_initial_model"]:
+            params = load_params(config["initial_model_path"], dev)                                   # ppo.py:246-248
+
+        rng, self.eval_rng = brandom.split(rng)
+        eval_env = BridgeBidding(table=eval_table, device=dev)
+        if eval_opp_params is None:
+            eval_opp_params = (load_params(config["eval_opp_model_path"], dev) if config["eval_opp_model_path"]
+                               else init_params(12345, dev))
+        self.simple_evaluate, self.simple_duplicate_evaluate, self.duplicate_evaluate = make_evaluators(config, eval_env,
+                                                                                                        eval_opp_params)
+
+        opp_forward_pass = make_fp(config["opp_activation"], config["opp_model_type"])
+        self.envs = [BridgeBidding(table=t, device=dev) for t in tables]                              # ppo.py:296-303
+        self.roll_outs = [make_roll_out(config, env, self.actor_forward_pass, opp_forward_pass) for env in self.envs]
+        self.calc_gae = make_calc_gae(config, self.actor_forward_pass)
+
+        rng, _rng = brandom.split(rng)
+        self.env, self.roll_out = self.envs[0], self.roll_outs[0]
+        env_state = self.env.init(self.env.make_keys(_rng, config["num_envs"]))
+        self.hash_index_list = np.arange(len(tables))
+        self.steps, self.hash_index, self.board_count = 0, 0, 0
+        terminated_count = torch.zeros((), dtype=torch.int64, device=dev)
+        rng, _rng = brandom.split(rng)
+        self.rng = rng
+        self.runner_state = (params, opt_state, env_state, env_state.observation, terminated_count, _rng)
+
+        if not config["self_play"]:
+            self.opp_params = load_params(config["opp_model_path"], dev) if config["opp_model_path"] else eval_opp_params
+        else:
+            self.opp_params = params
+        # past models.  ppo.py keeps them on disk (params-XXXXXXXX.pkl under save_model_path) and loads one at a time; here
+        # they only exist when the league can use them.  They are a zoo.ModelZoo packed in HBM (allocated once for every save
+        # the run makes, up to num_model_zoo): the PFSP probe is one league call and an opponent one device copy.  If that
+        # pool does not fit in free device memory at the start (after the zoos of the learners set up before this one), or
+        # when the opponent's forward is not the tensor-core one (which reads a packed opponent), they are host-memory NumPy
+        # dicts (14.7 MB each), copied to the device one at a time and probed one match each.
+        self.use_zoo = bool(config["self_play"]) and float(config["ratio_model_zoo"]) > 0.0
+        zoo_capacity = min(config["num_model_zoo"], max(0, config["num_updates"] - 1) // config["save_model_interval"])
+        self.zoo = []
+        probe_envs = config["num_prioritized_envs"] if config["prioritized_fictitious"] else 0
+        if self.use_zoo and isinstance(opp_forward_pass, ForwardPass) and device_zoo_fits(zoo_capacity, probe_envs, dev):
+            self.zoo = ModelZoo(zoo_capacity, dev)
+            if probe_envs:
+                self.pfsp_probe = make_device_pfsp_probe(eval_env, config["actor_activation"], config["actor_model_type"],
+                                                         probe_envs)
+                self.pfsp_probe.reserve(self.zoo)             # all of the zoo's device memory is taken here, once
+        self.device_zoo = isinstance(self.zoo, ModelZoo)
+        self.save_dir = os.path.join(config["log_path"], config["exp_name"], config["save_model_path"])
+        if config["save_model"]:
+            os.makedirs(self.save_dir, exist_ok=True)
+        self.logs = []
+
+    def zoo_model(self, k: int):
+        if self.device_zoo:
+            return self.zoo.opponent(k)
+        return {name: {kk: torch.as_tensor(v, device=self.dev) for kk, v in self.zoo[k][name].items()} for name in LAYERS}
+
+    def collect(self, i: int):
+        """Iteration i up to the update: saves, evaluations, opponent choice, rollout, GAE (ppo.py:351-477).  Returns
+        (traj_batch, advantages, targets) for the update step of self.runner_state."""
+        config, zoo, np_rng, eval_rng, dev = self.config, self.zoo, self.np_rng, self.eval_rng, self.dev
+        runner_state = self.runner_state
+        if i != 0 and i % config["save_model_interval"] == 0:                                      # ppo.py:351-362
+            if self.device_zoo:
+                zoo.append(runner_state[0])                  # keeps the newest zoo_capacity <= num_model_zoo models
+            elif self.use_zoo:
+                zoo.append(params_to_host(runner_state[0]))
+                zoo[:] = zoo[-config["num_model_zoo"]:]
+            if config["save_model"]:
+                save_params(runner_state[0], os.path.join(self.save_dir, f"params-{i:08}.pkl"))
+        t0 = time.time()
+        self.R = self.simple_evaluate(runner_state[0], eval_rng)                                  # ppo.py:365-368
+        self.eval_log = {}
+        if i % config["num_eval_step"] == 0:                                                      # ppo.py:369-374
+            log_info, _, _ = self.duplicate_evaluate(runner_state[0], eval_rng)
+            self.eval_log = make_evaluate_log(log_info)
+        self.t_eval = time.time() - t0
+
+        if config["self_play"]:                                                                   # ppo.py:376-470
+            (imp_opp, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng)
+            if imp_opp >= config["threshold_model_zoo"]:
+                if len(zoo) != 0 and np_rng.binomial(1, config["ratio_model_zoo"]):
+                    if config["prioritized_fictitious"]:
+                        imp_list = np.zeros(len(zoo))
+                        if self.device_zoo:  # the learner against every zoo model in one league call
+                            imp_list[:] = [imp for imp, _, _ in self.pfsp_probe(runner_state[0], zoo, eval_rng)]
+                        else:
+                            for k in range(len(zoo)):  # one past model on the device at a time
+                                (imp_list[k], _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.zoo_model(k),
+                                                                                              eval_rng)
+                        self.opp_params = self.zoo_model(int(np_rng.choice(len(zoo), p=pfsp_probabilities(imp_list,
+                                                                                                           config["prior_t"]))))
+                    else:
+                        self.opp_params = self.zoo_model(int(np_rng.integers(len(zoo))))
+                else:
+                    self.opp_params = runner_state[0]
+        (self.imp_opp_before, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng)
+        torch.cuda.synchronize(dev)
+        t1 = time.time()
+        runner_state, traj_batch = self.roll_out(runner_state, self.opp_params)                   # ppo.py:472-475
+        torch.cuda.synchronize(dev)
+        t2 = time.time()
+        advantages, targets = self.calc_gae(runner_state, traj_batch)                             # ppo.py:477
+        torch.cuda.synchronize(dev)
+        t3 = time.time()
+        self.t_rollout, self.t_gae = t2 - t1, t3 - t2
+        self.runner_state = runner_state
+        return traj_batch, advantages, targets
+
+    def finish_iteration(self, i: int, runner_state, loss_info, t_update: float) -> dict:
+        """Iteration i after the update (ppo.py:479-549): the strength probe, the log, the table rotation."""
+        config, dev = self.config, self.dev
+        self.runner_state = runner_state
+        (imp_opp_after, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, self.eval_rng)
+        self.steps += config["num_envs"] * config["num_steps"]
+        total_loss, (value_loss, loss_actor, entropy, approx_kl, clipflacs, illegal_action_loss) = loss_info
+        lr_now = self.optimizer.lr_at((i + 1) * config["update_epochs"] * config["num_minibatches"])
+        board_num = int(runner_state[4])
+        log = {                                                                                   # ppo.py:508-523
+            "train/score": float(self.R), "train/total_loss": float(total_loss[-1][-1]),
+            "train/value_loss": float(value_loss[-1][-1]), "train/loss_actor": float(loss_actor[-1][-1]),
+            "train/illegal_action_loss": float(illegal_action_loss[-1][-1]), "train/policy_entropy": float(entropy[-1][-1]),
+            "train/clipflacs": float(clipflacs[-1][-1]), "train/approx_kl": float(approx_kl[-1][-1]), "train/lr": lr_now,
+            "train/imp_opp_before": float(self.imp_opp_before), "train/imp_opp_after": float(imp_opp_after),
+            "board_num": board_num, "steps": self.steps,
+            "time/eval": self.t_eval, "time/rollout": self.t_rollout, "time/calc_gae": self.t_gae, "time/update": t_update,
+        }
+        log.update(self.eval_log)
+        self.logs.append(log)
+        if self.log_fn is not None:
+            self.log_fn(log)
+        if (board_num - self.board_count) // config["hash_size"] >= 1:                            # ppo.py:525-549
+            self.hash_index += 1
+            self.board_count = board_num
+            if self.hash_index == len(self.hash_index_list):
+                self.hash_index = 0
+                self.np_rng.shuffle(self.hash_index_list)
+            k = self.hash_index_list[self.hash_index]
+            self.env, self.roll_out = self.envs[k], self.roll_outs[k]
+            self.rng, _rng = brandom.split(self.rng)
+            env_state = self.env.init(self.env.make_keys(_rng, config["num_envs"]))
+            self.runner_state = (runner_state[0], runner_state[1], env_state, env_state.observation, runner_state[4], _rng)
+            log["table"] = int(k)
+        return log
+
+    def finish(self):
+        """The final save (ppo.py:550-569); -> (runner_state, logs) as `train` returns them."""
+        config = self.config
+        if config["save_model"]:
+            save_params(self.runner_state[0], os.path.join(self.save_dir, f"params-{config['num_updates']:08}.pkl"))
+            with open(os.path.join(self.save_dir, f"opt_state-{config['num_updates']:08}.pkl"), "wb") as fh:
+                st = self.runner_state[1]
+                pickle.dump({"count": st.count, "mu": st.mu.cpu().numpy(), "nu": st.nu.cpu().numpy()}, fh)
+        return self.runner_state, self.logs
+
+
 def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=None, device="cuda",
           log_fn: Optional[Callable[[dict], None]] = None, eval_opp_params=None, np_rng: Optional[np.random.Generator] = None,
           forward_pass_factory=None, update_step_factory=None):
     """`forward_pass_factory(activation, model_type)` / `update_step_factory(config, forward_pass, optimizer)` replace
     `make_forward_pass` / `make_update_step` -- the hook the cuBLAS cross-check (scripts/torch_baseline.py) plugs into;
     the defaults are the tensor-core kernels and nothing else."""
-    make_fp = forward_pass_factory or make_forward_pass
-    make_us = update_step_factory or make_update_step
-    cfg = dict(default_config())
-    cfg.update(config)
-    config = cfg
-    config["num_updates"] = config["total_timesteps"] // config["num_steps"] // config["num_envs"]   # ppo.py:225-227
-    config["num_minibatches"] = config["num_envs"] * config["num_steps"] // config["minibatch_size"]  # ppo.py:228-230
-    np_rng = np_rng or np.random.default_rng(config["seed"])
-    dev = torch.device(device)
-
-    def as_table(t):
-        return _deals.load_table(t) if isinstance(t, str) else np.asarray(t, dtype=np.uint8)
-
-    if tables is None:
-        d = config["dds_results_dir"]
-        if os.path.isdir(d):
-            tables = [os.path.join(d, f) for f in sorted(os.listdir(d)) if "train" in f]            # ppo.py:292-294
-            if eval_table is None and os.path.exists(os.path.join(d, "test_000.npy")):
-                eval_table = os.path.join(d, "test_000.npy")                                      # ppo.py:252
-        else:
-            tables = [_deals.synthetic_deal_table(config["hash_size"], seed=config["seed"] + k) for k in range(2)]
-    tables = [as_table(t) for t in tables]
-    eval_table = as_table(eval_table) if eval_table is not None else _deals.synthetic_deal_table(config["hash_size"], seed=10_000)
-
-    optimizer = make_optimizer(config)                                                            # ppo.py:195-211
-    actor_forward_pass = make_fp(config["actor_activation"], config["actor_model_type"])
-    rng, _rng = brandom.split(rng)
-    params = init_params(_rng & 0x7FFFFFFF, dev)                                                  # ppo.py:240-243
-    opt_state = optimizer.init(params)
-    if config["load_initial_model"]:
-        params = load_params(config["initial_model_path"], dev)                                   # ppo.py:246-248
-
-    rng, eval_rng = brandom.split(rng)
-    eval_env = BridgeBidding(table=eval_table, device=dev)
-    if eval_opp_params is None:
-        eval_opp_params = (load_params(config["eval_opp_model_path"], dev) if config["eval_opp_model_path"]
-                           else init_params(12345, dev))
-    simple_evaluate, simple_duplicate_evaluate, duplicate_evaluate = make_evaluators(config, eval_env, eval_opp_params)
-
-    opp_forward_pass = make_fp(config["opp_activation"], config["opp_model_type"])
-    envs = [BridgeBidding(table=t, device=dev) for t in tables]                                   # ppo.py:296-303
-    roll_outs = [make_roll_out(config, env, actor_forward_pass, opp_forward_pass) for env in envs]
-    calc_gae = make_calc_gae(config, actor_forward_pass)
-    update_step = make_us(config, actor_forward_pass, optimizer)
-
-    rng, _rng = brandom.split(rng)
-    env, roll_out = envs[0], roll_outs[0]
-    env_state = env.init(env.make_keys(_rng, config["num_envs"]))
-    hash_index_list = np.arange(len(tables))
-    steps, hash_index, board_count = 0, 0, 0
-    terminated_count = torch.zeros((), dtype=torch.int64, device=dev)
-    rng, _rng = brandom.split(rng)
-    runner_state = (params, opt_state, env_state, env_state.observation, terminated_count, _rng)
-
-    if not config["self_play"]:
-        opp_params = load_params(config["opp_model_path"], dev) if config["opp_model_path"] else eval_opp_params
-    else:
-        opp_params = params
-    # past models.  ppo.py keeps them on disk (params-XXXXXXXX.pkl under save_model_path) and loads one at a time; here they
-    # only exist when the league can use them.  They are a zoo.ModelZoo packed in HBM (allocated once for every save the run
-    # makes, up to num_model_zoo): the PFSP probe is one league call and an opponent one device copy.  If that pool does not
-    # fit in free device memory at the start, or when the opponent's forward is not the tensor-core one (which reads a packed
-    # opponent), they are host-memory NumPy dicts (14.7 MB each), copied to the device one at a time and probed one match
-    # each.
-    use_zoo = bool(config["self_play"]) and float(config["ratio_model_zoo"]) > 0.0
-    zoo_capacity = min(config["num_model_zoo"], max(0, config["num_updates"] - 1) // config["save_model_interval"])
-    zoo = []
-    probe_envs = config["num_prioritized_envs"] if config["prioritized_fictitious"] else 0
-    if use_zoo and isinstance(opp_forward_pass, ForwardPass) and device_zoo_fits(zoo_capacity, probe_envs, dev):
-        zoo = ModelZoo(zoo_capacity, dev)
-        if probe_envs:
-            pfsp_probe = make_device_pfsp_probe(eval_env, config["actor_activation"], config["actor_model_type"], probe_envs)
-            pfsp_probe.reserve(zoo)                          # all of the zoo's device memory is taken here, once
-    device_zoo = isinstance(zoo, ModelZoo)
-
-    def zoo_model(k: int):
-        if device_zoo:
-            return zoo.opponent(k)
-        return {name: {kk: torch.as_tensor(v, device=dev) for kk, v in zoo[k][name].items()} for name in LAYERS}
-    save_dir = os.path.join(config["log_path"], config["exp_name"], config["save_model_path"])
-    if config["save_model"]:
-        os.makedirs(save_dir, exist_ok=True)
-    logs = []
-    for i in range(config["num_updates"]):
-        if i != 0 and i % config["save_model_interval"] == 0:                                      # ppo.py:351-362
-            if device_zoo:
-                zoo.append(runner_state[0])                  # keeps the newest zoo_capacity <= num_model_zoo models
-            elif use_zoo:
-                zoo.append(params_to_host(runner_state[0]))
-                zoo[:] = zoo[-config["num_model_zoo"]:]
-            if config["save_model"]:
-                save_params(runner_state[0], os.path.join(save_dir, f"params-{i:08}.pkl"))
-        t0 = time.time()
-        R = simple_evaluate(runner_state[0], eval_rng)                                            # ppo.py:365-368
-        eval_log = {}
-        if i % config["num_eval_step"] == 0:                                                      # ppo.py:369-374
-            log_info, _, _ = duplicate_evaluate(runner_state[0], eval_rng)
-            eval_log = make_evaluate_log(log_info)
-        t_eval = time.time() - t0
-
-        if config["self_play"]:                                                                   # ppo.py:376-470
-            (imp_opp, _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], opp_params, eval_rng)
-            if imp_opp >= config["threshold_model_zoo"]:
-                if len(zoo) != 0 and np_rng.binomial(1, config["ratio_model_zoo"]):
-                    if config["prioritized_fictitious"]:
-                        imp_list = np.zeros(len(zoo))
-                        if device_zoo:  # the learner against every zoo model in one league call
-                            imp_list[:] = [imp for imp, _, _ in pfsp_probe(runner_state[0], zoo, eval_rng)]
-                        else:
-                            for k in range(len(zoo)):  # one past model on the device at a time
-                                (imp_list[k], _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], zoo_model(k),
-                                                                                         eval_rng)
-                        opp_params = zoo_model(int(np_rng.choice(len(zoo), p=pfsp_probabilities(imp_list, config["prior_t"]))))
-                    else:
-                        opp_params = zoo_model(int(np_rng.integers(len(zoo))))
-                else:
-                    opp_params = runner_state[0]
-        (imp_opp_before, _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], opp_params, eval_rng)
-        torch.cuda.synchronize(dev)
-        t1 = time.time()
-        runner_state, traj_batch = roll_out(runner_state, opp_params)                             # ppo.py:472-475
-        torch.cuda.synchronize(dev)
-        t2 = time.time()
-        advantages, targets = calc_gae(runner_state, traj_batch)                                  # ppo.py:477
-        torch.cuda.synchronize(dev)
+    learner = Learner(config, rng, tables, eval_table, device, log_fn, eval_opp_params, np_rng, forward_pass_factory)
+    update_step = (update_step_factory or make_update_step)(learner.config, learner.actor_forward_pass, learner.optimizer)
+    for i in range(learner.config["num_updates"]):
+        traj_batch, advantages, targets = learner.collect(i)
         t3 = time.time()
-        runner_state, loss_info = update_step(runner_state, traj_batch, advantages, targets)     # ppo.py:479-484
+        runner_state, loss_info = update_step(learner.runner_state, traj_batch, advantages, targets)  # ppo.py:479-484
+        torch.cuda.synchronize(learner.dev)
+        learner.finish_iteration(i, runner_state, loss_info, time.time() - t3)
+    return learner.finish()
+
+
+def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optional[Sequence] = None, eval_table=None,
+                     device="cuda", log_fns: Optional[Sequence[Optional[Callable[[dict], None]]]] = None,
+                     eval_opp_params=None, np_rngs: Optional[Sequence[Optional[np.random.Generator]]] = None):
+    """`train` for K learners on one GPU.  Each learner runs its own control plane (evaluations, FSP / PFSP opponents and
+    zoo, rollout, GAE, logging, table rotation) in turn, and the K updates of an iteration run as one grouped update step
+    (update.make_population_update_step), so that the learners' GEMM tiles share the device.  configs[k] and rngs[k] give
+    learner k exactly the run `train(configs[k], rngs[k], ...)` gives; the keys of update.POPULATION_SHARED_KEYS must be
+    equal across learners (ValueError naming the first that is not).  -> [(runner_state, logs)] per learner."""
+    K = len(configs)
+    if len(rngs) != K:
+        raise ValueError("train_population needs one rng per config")
+    full = [full_config(c) for c in configs]
+    check_population_configs(full)
+    log_fns = list(log_fns) if log_fns is not None else [None] * K
+    np_rngs = list(np_rngs) if np_rngs is not None else [None] * K
+    learners = [Learner(configs[k], rngs[k], tables, eval_table, device, log_fns[k], eval_opp_params, np_rngs[k]) for k in range(K)]
+    update_step = make_population_update_step([ln.config for ln in learners], learners[0].actor_forward_pass,
+                                              [ln.optimizer for ln in learners])
+    dev = learners[0].dev
+    for i in range(full[0]["num_updates"]):
+        batches = [ln.collect(i) for ln in learners]
+        t3 = time.time()
+        outs = update_step([ln.runner_state for ln in learners], [b[0] for b in batches], [b[1] for b in batches],
+                           [b[2] for b in batches])
         torch.cuda.synchronize(dev)
-        t4 = time.time()
-        (imp_opp_after, _, _), _, _, _ = simple_duplicate_evaluate(runner_state[0], opp_params, eval_rng)
-        steps += config["num_envs"] * config["num_steps"]
-        total_loss, (value_loss, loss_actor, entropy, approx_kl, clipflacs, illegal_action_loss) = loss_info
-        lr_now = optimizer.lr_at((i + 1) * config["update_epochs"] * config["num_minibatches"])
-        board_num = int(runner_state[4])
-        log = {                                                                                   # ppo.py:508-523
-            "train/score": float(R), "train/total_loss": float(total_loss[-1][-1]),
-            "train/value_loss": float(value_loss[-1][-1]), "train/loss_actor": float(loss_actor[-1][-1]),
-            "train/illegal_action_loss": float(illegal_action_loss[-1][-1]), "train/policy_entropy": float(entropy[-1][-1]),
-            "train/clipflacs": float(clipflacs[-1][-1]), "train/approx_kl": float(approx_kl[-1][-1]), "train/lr": lr_now,
-            "train/imp_opp_before": float(imp_opp_before), "train/imp_opp_after": float(imp_opp_after),
-            "board_num": board_num, "steps": steps,
-            "time/eval": t_eval, "time/rollout": t2 - t1, "time/calc_gae": t3 - t2, "time/update": t4 - t3,
-        }
-        log.update(eval_log)
-        logs.append(log)
-        if log_fn is not None:
-            log_fn(log)
-        if (board_num - board_count) // config["hash_size"] >= 1:                                 # ppo.py:525-549
-            hash_index += 1
-            board_count = board_num
-            if hash_index == len(hash_index_list):
-                hash_index = 0
-                np_rng.shuffle(hash_index_list)
-            env, roll_out = envs[hash_index_list[hash_index]], roll_outs[hash_index_list[hash_index]]
-            rng, _rng = brandom.split(rng)
-            env_state = env.init(env.make_keys(_rng, config["num_envs"]))
-            runner_state = (runner_state[0], runner_state[1], env_state, env_state.observation, runner_state[4], _rng)
-            log["table"] = int(hash_index_list[hash_index])
-    if config["save_model"]:                                                                      # ppo.py:550-569
-        save_params(runner_state[0], os.path.join(save_dir, f"params-{config['num_updates']:08}.pkl"))
-        with open(os.path.join(save_dir, f"opt_state-{config['num_updates']:08}.pkl"), "wb") as fh:
-            st = runner_state[1]
-            pickle.dump({"count": st.count, "mu": st.mu.cpu().numpy(), "nu": st.nu.cpu().numpy()}, fh)
-    return runner_state, logs
+        t_update = time.time() - t3
+        for ln, (runner_state, loss_info) in zip(learners, outs):
+            ln.finish_iteration(i, runner_state, loss_info, t_update)
+    return [ln.finish() for ln in learners]

@@ -12,9 +12,9 @@ from __future__ import annotations
 
 import torch
 
-from . import ops
+from . import _lib, ops
 from . import random as brandom
-from .optim import OptState, flatten_params
+from .optim import OptState, flatten_params, update_mlp_grouped_
 
 _STAT_NAMES = ("total_loss", "value_loss", "loss_actor", "entropy", "approx_kl", "clipflacs", "illegal_action_loss")
 
@@ -93,5 +93,131 @@ def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None)
                              **cfg)                                                # src/update.py:164-167
                 state = optimizer.update_mlp_(flat_p, flat_g, state, acc[14:15], blob)  # src/update.py:168-169
         return finish()
+
+    return update_step
+
+
+# Keys every learner of a population must share: they fix the shapes of the stacked buffers and the flags and tile widths
+# of the grouped launches (brl_ppo_grad_grouped).  Everything else -- seed, lr, anneal_lr, the loss coefficients,
+# max_grad_norm, gamma, gae_lambda, opponents -- may differ per learner.
+POPULATION_SHARED_KEYS = ("num_envs", "num_steps", "minibatch_size", "update_epochs", "total_timesteps",
+                          "actor_illegal_action_mask", "value_clipping", "reward_scaling", "global_gradient_clipping",
+                          "illegal_action_loss_stat", "actor_model_type", "actor_activation", "brl_train_tune")
+
+
+def check_population_configs(configs) -> None:
+    """ValueError naming the first key of POPULATION_SHARED_KEYS on which two learners' configs differ."""
+    if not configs:
+        raise ValueError("a population needs at least one learner")
+    _missing = object()
+    for key in POPULATION_SHARED_KEYS:
+        values = [c.get(key, _missing) for c in configs]
+        if any(v != values[0] for v in values[1:]):
+            raise ValueError(f"population learners must share config[{key!r}]; got {[None if v is _missing else v for v in values]}")
+
+
+def make_population_update_step(configs, actor_forward_pass, optimizers, permutation_fn=None):
+    """`make_update_step` for K learners whose optimizer steps run as one grouped step (ops.ppo_grad_grouped,
+    optim.update_mlp_grouped_).  update_step(runner_states, traj_batches, advantages, targets) takes one entry per
+    learner and returns K `(runner_state, loss_info)` pairs, each what `make_update_step(configs[k], ...)` returns for
+    that learner: every learner draws its permutations from its own key, and its parameters, optimizer state and loss
+    statistics are bit-identical to its solo update.  The stacked parameter, gradient, moment and blob buffers of the
+    whole update are owned here; the returned params / opt_state are views into them."""
+    configs = list(configs)
+    check_population_configs(configs)
+    if len(optimizers) != len(configs):
+        raise ValueError("make_population_update_step needs one optimizer per config")
+    if len(configs) > _lib.MAX_LEARNERS:
+        raise ValueError(f"a population has at most {_lib.MAX_LEARNERS} learners")
+    c0 = configs[0]
+    masked = bool(c0["actor_illegal_action_mask"])
+    flags = dict(value_clipping=bool(c0.get("value_clipping", True)), reward_scaling=bool(c0.get("reward_scaling", False)),
+                 masked_policy=masked)
+    coef_rows = [[float(c["clip_eps"]), float(c["ent_coef"]), float(c["vf_coef"]), float(c.get("illegal_action_l2norm_coef", 0.0))]
+                 for c in configs]
+    stat_mode = c0.get("illegal_action_loss_stat", "last")
+    if stat_mode not in ("last", "all"):
+        raise ValueError("illegal_action_loss_stat must be 'last' or 'all'")
+    if getattr(actor_forward_pass, "precision", None) not in ("tc", "tc-bf16"):
+        raise TypeError("make_population_update_step needs a brl_b200.models.ForwardPass (tensor-core ReLU net)")
+    tune = int(c0.get("brl_train_tune", 0))
+    K = len(configs)
+
+    def default_permutation(rng, batch_size, device):
+        g = torch.Generator(device="cpu").manual_seed(rng & 0x7FFFFFFFFFFFFFFF)
+        return torch.randperm(batch_size, generator=g).to(device=device, dtype=torch.int32)
+
+    def update_step(runner_states, traj_batches, advantages, targets):
+        if not (len(runner_states) == len(traj_batches) == len(advantages) == len(targets) == K):
+            raise ValueError(f"update_step needs {K} runner states, trajectories, advantages and targets")
+        dev = advantages[0].device
+        nmb, mbs = int(c0["num_minibatches"]), int(c0["minibatch_size"])
+        batch_size = nmb * mbs
+        n_epochs = int(c0["update_epochs"])
+        flat = []  # per learner: the ppo_grad buffers of its flat rollout (src/update.py:195-197)
+        obs_dtype = None
+        for tb, adv, tgt in zip(traj_batches, advantages, targets):
+            T, n = adv.shape
+            assert batch_size == T * n, "batch size must be equal to number of steps * number of envs"
+            obs = tb.obs.reshape(batch_size, -1)
+            if obs.dtype == torch.bool:
+                obs = obs.view(torch.uint8)
+            if obs_dtype is not None and obs.dtype != obs_dtype:
+                raise ValueError("population learners must record observations of one dtype")
+            obs_dtype = obs.dtype
+            flat.append((obs.contiguous(), tb.legal_action_mask.reshape(batch_size, -1).view(torch.uint8).contiguous(),
+                         tb.action.reshape(batch_size).contiguous(), tb.log_prob.reshape(batch_size).contiguous(),
+                         tb.value.reshape(batch_size).contiguous(), adv.reshape(batch_size).contiguous(),
+                         tgt.reshape(batch_size).contiguous()))
+
+        n_params, blob_bytes = ops.mlp_num_params(), int(_lib.load().brl_mlp_train_blob_bytes())
+        flat_p = torch.zeros((K, ops.mlp_param_stride()), dtype=torch.float32, device=dev)  # learner k: flat_p[k, :n_params]
+        m = torch.zeros_like(flat_p)
+        v = torch.zeros_like(flat_p)
+        blob = torch.empty((K, blob_bytes), dtype=torch.uint8, device=dev)
+        new_params, states, rngs, rest = [], [], [], []
+        for k, (rs, opt) in enumerate(zip(runner_states, optimizers)):
+            params, opt_state, env_state, last_obs, terminated_count, rng = rs
+            _, p_k = flatten_params(params, out=flat_p[k, :n_params])
+            if opt_state is None:
+                opt_state = opt.init(params)
+            m[k, :n_params].copy_(opt_state.mu)
+            v[k, :n_params].copy_(opt_state.nu)
+            ops.mlp_pack_train(flat_p[k, :n_params], out=blob[k])
+            new_params.append(p_k)
+            states.append(OptState(opt_state.count, m[k, :n_params], v[k, :n_params]))
+            rngs.append(rng)
+            rest.append((env_state, last_obs, terminated_count))
+        flat_g = torch.zeros_like(flat_p)
+        stats_all = torch.zeros((n_epochs, nmb, K, 8), dtype=torch.float32, device=dev)
+        acc = torch.zeros((K, _lib.PPO_SCRATCH_BYTES // 8), dtype=torch.float64, device=dev)
+        scratch = torch.empty(ops.ppo_grad_grouped_scratch_bytes(K, mbs), dtype=torch.uint8, device=dev)
+        coefs = torch.tensor(coef_rows, dtype=torch.float32).to(dev)
+
+        def permutation(_rng):
+            return (permutation_fn(_rng, batch_size) if permutation_fn is not None
+                    else default_permutation(_rng, batch_size, dev)).to(device=dev, dtype=torch.int32).contiguous()
+
+        for epoch in range(n_epochs):
+            perms = []
+            for k in range(K):
+                rngs[k], _rng = brandom.split(rngs[k])                            # src/update.py:187
+                perms.append(permutation(_rng))
+            # this epoch's trajectory tables, one [K, 8] per minibatch: the index column steps through each permutation
+            base = torch.tensor([ops.ppo_trajectory_row(f[0], perms[k], *f[1:]) for k, f in enumerate(flat)], dtype=torch.int64)
+            tables = base.repeat(nmb, 1, 1)
+            tables[:, :, 1] += torch.arange(nmb, dtype=torch.int64)[:, None] * (4 * mbs)  # int32 index: 4 bytes a row
+            tables = tables.pin_memory().to(dev, non_blocking=True)
+            for mb in range(nmb):
+                ops.ppo_grad_grouped(tables[mb], coefs, blob, scratch, flat_g, stats_all[epoch, mb], acc, batch=mbs,
+                                     obs_dtype=obs_dtype, illegal_stat=stat_mode == "all" or mb == nmb - 1, tune=tune, **flags)
+                states = update_mlp_grouped_(optimizers, flat_p, flat_g, m, v, states, acc, blob)
+
+        out = []
+        for k in range(K):
+            cols = [stats_all[:, :, k, i] for i in range(7)]
+            env_state, last_obs, terminated_count = rest[k]
+            out.append(((new_params[k], states[k], env_state, last_obs, terminated_count, rngs[k]), (cols[0], tuple(cols[1:]))))
+        return out
 
     return update_step

@@ -53,6 +53,7 @@
  *                         take + forward + loss + backward through the MLP on tcgen05   src/update.py:91-167,194-199
  *   brl_mlp_pack_train    flat fp32 params -> device layout for brl_ppo_grad
  *   brl_mlp_adam_step     optimizer.update + apply_updates + refresh of that layout, one pass   src/update.py:168-169
+ *   brl_ppo_grad_grouped / brl_mlp_adam_step_grouped   the two above for K learners at once (population training)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -463,6 +464,43 @@ int32_t brl_mlp_adam_step(brl_stream_t, void **buffers, const void *opaque, size
  *               element 14 = sum of squares of grads (the input of brl_adam_apply) */
 int32_t brl_ppo_grad(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- population training: one optimizer step of K learners in the launches of one ------------------------------------
+ * K PPO learners of the same shape (minibatch size B, flags) each take their step on their own weights, trajectory and
+ * coefficients.  The GEMM tiles of all learners share one fused forward and one fused backward launch, so that one
+ * learner's dependency gaps are filled by the others' tiles.  Learner k's gradient, stats and |g|^2 are bit-identical to
+ * a brl_ppo_grad call with its inputs (same tile widths, K-block order and epilogue arithmetic); its |g|^2 is a sum of
+ * f64 atomics and may differ in the last bits.  An empty batch (n_learners = 0 or batch = 0) is a no-op and its buffers
+ * may be NULL. */
+#define BRL_MAX_LEARNERS 64
+/* floats between two learners' rows of a population's flat parameter / gradient / moment buffers [K, stride]: the row
+ * is brl_mlp_num_params() floats padded to 256 bytes (the padding is neither read nor written) */
+int64_t brl_mlp_param_stride(void);
+typedef struct BrlPpoGroupedParams {
+    int64_t batch;         /* samples in each learner's minibatch (one B for all)                                        */
+    int32_t n_learners;    /* K, 0 .. BRL_MAX_LEARNERS                                                                   */
+    int32_t flags;         /* BRL_PPO_* incl. BRL_PPO_OBS_*, the same for all learners                                    */
+    int32_t reserved;      /* 0; bits 2 / 4 pick the fused launches' tile widths as in BrlPpoParams.reserved (bit 3 unused) */
+    int32_t pad;           /* 0 */
+} BrlPpoGroupedParams;
+int64_t brl_ppo_grad_grouped_scratch_bytes(int64_t n_learners, int64_t batch);
+/* brl_ppo_grad for K learners.  opaque = BrlPpoGroupedParams.  Learner k's rows of a [K, ...] buffer are its own.
+ * buffers: [0] in i64 traj[K, 8]: device addresses of learner k's obs[total_k, 480] (dtype per BRL_PPO_OBS_*), i32 index[B]
+ *              (NULL = identity), u8 mask[total_k, 38], i32 action, f32 old_log_prob, old_value, advantages, targets [total_k]
+ *              -- the buffers of brl_ppo_grad, one allocation per learner; 16-byte aligned table
+ *          [1] in f32 coefs[K, 4] = {clip_eps, ent_coef, vf_coef, illegal_l2_coef} per learner
+ *          [2] in blob[K, brl_mlp_train_blob_bytes()]  [3] scratch[brl_ppo_grad_grouped_scratch_bytes(K, B)]
+ *          [4] out f32 grads[K, brl_mlp_param_stride()]  [5] out f32 stats[K, 8] (as brl_ppo_grad)
+ *          [6] scratch acc[K, BRL_PPO_SCRATCH_BYTES]; on return learner k's f64 element 14 = its |grads|^2
+ * Buffers [2], [3], [4] and [6] are 16-byte aligned.  Undefined: a table address that is not a valid buffer of the size
+ * above, an index outside [0, total_k), buffers that overlap. */
+int32_t brl_ppo_grad_grouped(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_mlp_adam_step for K learners in one launch.  opaque = BrlAdamParams[K] (opaque_len = K * sizeof, 0 = no-op): learner
+ * k's step count, learning rate, betas, eps and max_grad_norm; n = brl_mlp_num_params() for every k.
+ * buffers: [0] inout f32 params[K, s]  [1] in f32 grads[K, s]  [2] inout f32 m[K, s]  [3] inout f32 v[K, s], s =
+ *              brl_mlp_param_stride()  [4] in acc[K, BRL_PPO_SCRATCH_BYTES] of brl_ppo_grad_grouped (learner k's |grads|^2: its f64 element 14)
+ *          [5] inout blob[K, brl_mlp_train_blob_bytes()]; all 16-byte aligned */
+int32_t brl_mlp_adam_step_grouped(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- supervised bidding pre-training (sl.py): examples from stored auctions, cross-entropy step ---------------------- */
 /* Examples of the OpenSpiel bidding data (sl.py:87-117): one deal row per trajectory (deals.py format, DD nibbles unused),
  * dealer North, nobody vulnerable, players = seats (bridge(use_double_dummy_result=false), sl.py:44).  The calls of
@@ -574,6 +612,8 @@ void brl_gather_rows_xla(brl_stream_t, void **buffers, const char *opaque, size_
 void brl_mlp_pack_train_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_mlp_adam_step_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_ppo_grad_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_mlp_adam_step_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_act_log_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_summary_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_sl_examples_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);

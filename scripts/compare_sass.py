@@ -8,9 +8,9 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES records the grouped-forward change: the host-count grouped instantiations (k_mlp_layer / k_mlp_fused with
-GROUPED = true and DEVCOUNT = false, k_gather_obs_rows<true>) are gone, the <GROUPED, DEVCOUNT> pair became one GROUPED flag,
-and the device-count gather was renamed.  Replace the table for another change."""
+RENAMES records the population-training change: k_train_fused gained a GROUPED flag (the solo kernels are GROUPED = false)
+and k_ppo_prepass / k_ppo_loss became templates over their argument type (the solo kernels take PpoArgs),
+and ADDED lists the grouped kernels it adds.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -19,13 +19,16 @@ import sys
 from collections import OrderedDict
 
 RENAMES = [  # demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-    (r"^brl::k_mlp_layer<\(int\)\d+(, \(bool\)[01]){3}, \(bool\)1, \(bool\)0>$", None),
-    (r"^(brl::k_mlp_layer<\(int\)\d+(?:, \(bool\)[01]){3}), (\(bool\)[01]), \2>$", r"\1, \2>"),
-    (r"^brl::k_mlp_fused<\(bool\)[01], \(bool\)1, \(bool\)0>$", None),
-    (r"^(brl::k_mlp_fused<\(bool\)[01]), (\(bool\)[01]), \2>$", r"\1, \2>"),
-    (r"^brl::k_gather_obs_rows<\(bool\)1>$", None),
-    (r"^brl::k_gather_obs_rows<\(bool\)0>$", "brl::k_gather_obs_rows"),
-    (r"^brl::k_gather_obs_rows_dev$", "brl::k_gather_obs_rows_grouped"),
+    (r"^brl::k_train_fused<\(int\)(\d+)>$", r"brl::k_train_fused<(int)\1, (bool)0>"),
+    (r"^brl::k_ppo_(prepass|loss)$", r"brl::k_ppo_\1<brl::PpoArgs>"),
+]
+ADDED = [  # kernels the change adds on purpose: reported, not counted as unexpected
+    r"^brl::k_train_fused<\(int\)\d+, \(bool\)1>$",
+    r"^brl::k_gather_obs_grouped<.*>$",
+    r"^brl::k_bias_grad_grouped$",
+    r"^brl::k_adam_pack_grouped$",
+    r"^brl::k_ppo_(prepass|loss)<brl::PpoGroupArgs>$",
+    r"^brl::k_ppo_gram_grouped$",
 ]
 
 
@@ -63,7 +66,7 @@ def _split(text, head):
         if line.startswith("Fatbin"):
             cur = None
         elif cur is not None and line.strip():
-            funcs[cur].append(line.strip())
+            funcs[cur].append(" ".join(line.split()))  # cuobjdump pads columns to the listing's longest line
     return funcs
 
 
@@ -116,10 +119,16 @@ def main(argv=None):
             bad += 1
             what = "SASS" if got[0] != body else "resources"
             lines.append(f"DIFFERENT  {tu}  {name} -> {target}  ({what})  old [{res}] new [{got[1]}]")
+    added = 0
     for key in sorted(set(new) - matched):
-        bad += 1
-        lines.append(f"ADDED      {key[0]}  {key[1]}  [{new[key][1]}]")
-    lines.append(f"{len(old)} kernels before, {len(new)} after: {same} identical, {removed} removed as intended, {bad} unexpected")
+        if any(re.match(pat, key[1]) for pat in ADDED):
+            added += 1
+            lines.append(f"added      {key[0]}  {key[1]}  [{new[key][1]}]")
+        else:
+            bad += 1
+            lines.append(f"ADDED      {key[0]}  {key[1]}  [{new[key][1]}]")
+    lines.append(f"{len(old)} kernels before, {len(new)} after: {same} identical, {removed} removed as intended, {added} added as intended, "
+                 f"{bad} unexpected")
     report = "\n".join(lines) + "\n"
     sys.stdout.write(report)
     if a.out:
