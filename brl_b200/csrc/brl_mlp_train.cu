@@ -946,6 +946,20 @@ using namespace brl;
 
 static int train_ops(OpSpec* fwd, OpSpec* bwd, unsigned char* sc, const unsigned char* blob, float* grads, double* grad_sumsq, int B);
 
+// one learner's BrlAdamParams -> the optimizer scalars of AdamPackArgs / AdamLearner (learner < 0: a solo step)
+template <class D>
+static int32_t adam_scalars(const char* what, long long learner, const BrlAdamParams& p, D& d) {
+    if (p.n != (int64_t)flat_layout().total || p.step <= 0) {
+        char at[32] = "";
+        if (learner >= 0) snprintf(at, sizeof(at), "learner %lld: ", learner);
+        return fail(BRL_E_OPAQUE, "%s: %sn must be brl_mlp_num_params() and step (1-based) > 0", what, at);
+    }
+    d.max_norm = p.max_grad_norm; d.lr = p.lr; d.b1 = p.beta1; d.b2 = p.beta2; d.eps = p.eps;
+    d.bc1 = 1.0f - powf(p.beta1, (float)p.step);
+    d.bc2 = 1.0f - powf(p.beta2, (float)p.step);
+    return BRL_OK;
+}
+
 extern "C" {
 
 int64_t brl_mlp_num_params(void) { return (int64_t)flat_layout().total; }
@@ -981,24 +995,16 @@ int32_t brl_mlp_pack_train(brl_stream_t stream, void** b, const void* opaque, si
 int32_t brl_mlp_adam_step(brl_stream_t stream, void** b, const void* opaque, size_t len) {
     if (opaque == nullptr || len != sizeof(BrlAdamParams))
         return fail(BRL_E_OPAQUE, "brl_mlp_adam_step: opaque must be one BrlAdamParams (%zu bytes), got %zu", sizeof(BrlAdamParams), len);
-    const BrlAdamParams* p = static_cast<const BrlAdamParams*>(opaque);
     static const char* names[] = {"params", "grads", "m", "v", "sumsq", "blob"};
-    for (int k = 0; k < 6; ++k) {
-        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_mlp_adam_step: buffer '%s' is NULL", names[k]);
-        if (k != 4 && (reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_mlp_adam_step: buffer '%s' is not 16-byte aligned", names[k]);
-    }
-    if (p->n != (int64_t)flat_layout().total || p->step <= 0)
-        return fail(BRL_E_OPAQUE, "brl_mlp_adam_step: n must be brl_mlp_num_params() and step (1-based) > 0");
     AdamPackArgs a{};
+    int32_t rc = check_buffers("brl_mlp_adam_step", b, names, 6, 0, 0x3Fu & ~(1u << 4));
+    if (rc != BRL_OK || (rc = adam_scalars("brl_mlp_adam_step", -1, *static_cast<const BrlAdamParams*>(opaque), a)) != BRL_OK) return rc;
     a.p = static_cast<float*>(b[0]);
     a.g = static_cast<const float*>(b[1]);
     a.m = static_cast<float*>(b[2]);
     a.v = static_cast<float*>(b[3]);
     a.sumsq = static_cast<const double*>(b[4]);
     a.blob = static_cast<unsigned char*>(b[5]);
-    a.max_norm = p->max_grad_norm; a.lr = p->lr; a.b1 = p->beta1; a.b2 = p->beta2; a.eps = p->eps;
-    a.bc1 = 1.0f - powf(p->beta1, (float)p->step);
-    a.bc2 = 1.0f - powf(p->beta2, (float)p->step);
     a.F = flat_layout();
     a.T = train_blob();
     launch_pdl(k_adam_pack<true>, dim3(adam_pack_grid()), dim3(256), 0, (cudaStream_t)stream, a);
@@ -1012,10 +1018,8 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
     if (p->batch <= 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "brl_ppo_grad: batch must be in [1, 2^24]");
     static const char* names[] = {"obs", "blob", "scratch", "index", "mask", "action", "old_log_prob", "old_value", "advantages",
                                   "targets", "grads", "stats", "acc"};
-    for (int k = 0; k < 13; ++k)
-        if (b[k] == nullptr && k != 3) return fail(BRL_E_BUFFER, "brl_ppo_grad: buffer '%s' is NULL", names[k]);
-    for (int k : {0, 1, 2, 10})
-        if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_ppo_grad: buffer '%s' is not 16-byte aligned", names[k]);
+    const int32_t rc = check_buffers("brl_ppo_grad", b, names, 13, 1u << 3, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 10);
+    if (rc != BRL_OK) return rc;
     if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad: cuTensorMapEncodeTiled not available from the driver");
     cudaStream_t s = (cudaStream_t)stream;
     // 3. loss head + its backward (src/update.py:97-162)
@@ -1066,11 +1070,10 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
 // scratch: K per-learner minibatch scratches (train_scratch(B), learner k's at k * total), then the grouped launches' tile
 // counters: [2 launches][kMaxOps][K][nmb + 1]
 static size_t grouped_ready_offset(int64_t K, int64_t B) { return (size_t)K * train_scratch(B).total; }
-static size_t grouped_ready_words(int64_t K, int64_t B) { return (size_t)2 * kMaxOps * K * (size_t)(ready_blocks(B) + 1); }
 
 int64_t brl_ppo_grad_grouped_scratch_bytes(int64_t n_learners, int64_t batch) {
     if (n_learners <= 0 || batch <= 0 || n_learners > BRL_MAX_LEARNERS || batch > (1 << 24)) return 0;
-    return (int64_t)(grouped_ready_offset(n_learners, batch) + grouped_ready_words(n_learners, batch) * sizeof(uint32_t));
+    return (int64_t)(grouped_ready_offset(n_learners, batch) + n_learners * ready_words(batch) * sizeof(uint32_t));
 }
 
 int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -1083,104 +1086,39 @@ int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, 
     if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: batch must be in [0, 2^24]");
     if (p->n_learners == 0 || p->batch == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL
     static const char* names[] = {"traj", "coefs", "blob", "scratch", "grads", "stats", "acc"};
-    for (int k = 0; k < 7; ++k)
-        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_ppo_grad_grouped: buffer '%s' is NULL", names[k]);
-    for (int k : {0, 2, 3, 4, 6})
-        if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_ppo_grad_grouped: buffer '%s' is not 16-byte aligned", names[k]);
+    const int32_t rc = check_buffers("brl_ppo_grad_grouped", b, names, 7, 0, 1u << 0 | 1u << 2 | 1u << 3 | 1u << 4 | 1u << 6);
+    if (rc != BRL_OK) return rc;
     if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad_grouped: cuTensorMapEncodeTiled not available from the driver");
-    cudaStream_t s = (cudaStream_t)stream;
-    const char* what = "brl_ppo_grad_grouped";
-    const int K = p->n_learners, B = (int)p->batch;
-    const TrainScratch S = train_scratch(B);
-    const TrainBlob T = train_blob();
-    const FlatLayout F = flat_layout();
-    const long long* traj = static_cast<const long long*>(b[0]);
-    const float* coefs = static_cast<const float*>(b[1]);
-    const unsigned char* blob = static_cast<const unsigned char*>(b[2]);
-    unsigned char* sc = static_cast<unsigned char*>(b[3]);
-    float* grads = static_cast<float*>(b[4]);
-    float* stats = static_cast<float*>(b[5]);
-    unsigned char* acc = static_cast<unsigned char*>(b[6]);
-    double* grad_sumsq = reinterpret_cast<double*>(acc) + 14;  // learner k's |g|^2: f64 14 of its accumulator slice
-    const bool illegal_stat = (p->flags & BRL_PPO_ILLEGAL_STAT) != 0;
-    const int nmb = ready_blocks(B);
-    uint32_t* ready = reinterpret_cast<uint32_t*>(sc + grouped_ready_offset(K, B));
-    int32_t rc = BRL_OK;
-
-    // 0. tile counters and every learner's f64 accumulators
-    if (cudaMemsetAsync(ready, 0, grouped_ready_words(K, B) * sizeof(uint32_t), s) != cudaSuccess ||
-        cudaMemset2DAsync(acc, BRL_PPO_SCRATCH_BYTES, 0, 16 * sizeof(double), (size_t)K, s) != cudaSuccess)
-        return check_launch(what);
-    // 1. every learner's minibatch of observations
-    {
-        const dim3 grid((unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256), (unsigned)K);
-        uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
-        const long long st = (long long)S.total;
-        if (p->flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs_grouped<__nv_bfloat16>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
-        else if (p->flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs_grouped<uint8_t>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
-        else launch_pdl(k_gather_obs_grouped<float>, grid, dim3(256), 0, s, traj, (int64_t)B, o, st);
-    }
-    // 2. the forward GEMMs of all learners as one launch, described by learner 0's ops: A operands (activations, dz) lie in
-    //    the scratch, B operands in the blob (forward, dgrad) or the scratch (wgrad)
-    OpSpec fwd[5], bwd[kMaxOps];
-    const int nb = train_ops(fwd, bwd, sc, blob, grads, grad_sumsq, B);
-    const GroupSpec grp{K, (long long)S.total, (long long)T.total, (long long)param_stride(), BRL_PPO_SCRATCH_BYTES / (long long)sizeof(double)};
-    for (OpSpec* o : {fwd + 0, fwd + 1, fwd + 2, fwd + 3, fwd + 4}) { o->a_stride = grp.sc_stride; o->w_stride = grp.blob_stride; }
-    for (int i = 0; i < nb; ++i) {
-        bwd[i].a_stride = grp.sc_stride;
-        bwd[i].w_stride = bwd[i].epi == kEpiWgrad ? grp.sc_stride : grp.blob_stride;
-    }
-    const int tune = p->reserved;
-    const bool wide_fwd = (tune & 4) != 0, wide_bwd = (tune & 16) == 0;  // the tile widths of launch_train_minibatch
-    rc = wide_fwd ? launch_fused_ops<128, true>(s, fwd, 5, nmb, ready, nullptr, what, &grp)
-                  : launch_fused_ops<64, true>(s, fwd, 5, nmb, ready, nullptr, what, &grp);
-    if (rc != BRL_OK) return rc;
-    if ((rc = check_launch(what)) != BRL_OK) return rc;
-    // 3. the loss heads
-    PpoGroupIO io{};
-    io.traj = traj;
-    io.coefs = coefs;
-    io.head.logits = reinterpret_cast<const float*>(sc + S.logits);
-    io.head.value = reinterpret_cast<const float*>(sc + S.value);
-    io.head.dlogits = reinterpret_cast<float*>(sc + S.dlogits);
-    io.head.dvalue = reinterpret_cast<float*>(sc + S.dvalue);
-    io.head.dz_hi = sc + S.dz5_hi;
-    io.head.dz_lo = sc + S.dz5_lo;
-    io.sc_stride = (long long)S.total;
-    io.stats = stats;
-    io.acc = acc;
-    io.batch = B;
-    io.K = K;
+    PpoGroupIO io{};  // the loss heads' arguments but the forward outputs, which launch_train_minibatch hands to the head
+    io.traj = static_cast<const long long*>(b[0]);
+    io.coefs = static_cast<const float*>(b[1]);
+    io.sc_stride = (long long)train_scratch(p->batch).total;
+    io.stats = static_cast<float*>(b[5]);
+    io.acc = static_cast<unsigned char*>(b[6]);
+    io.batch = p->batch;
+    io.K = p->n_learners;
     io.flags = p->flags & (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
-    if ((rc = launch_ppo_loss_grouped(s, io)) != BRL_OK) return rc;
-    // 4. the backward GEMMs
-    uint32_t* ready_bwd = ready + (size_t)kMaxOps * K * (nmb + 1);
-    rc = wide_bwd ? launch_fused_ops<128, true>(s, bwd, nb, nmb, ready_bwd, nullptr, what, &grp)
-                  : launch_fused_ops<64, true>(s, bwd, nb, nmb, ready_bwd, nullptr, what, &grp);
-    if (rc != BRL_OK) return rc;
-    // 5. bias gradients (and the deferred illegal-action statistics)
-    {
-        GroupedBiasArgs g{};
-        for (int l = 0; l < 4; ++l) {
-            g.a.hi[l] = reinterpret_cast<const __nv_bfloat16*>(sc + S.dz_hi[l]);
-            g.a.lo[l] = reinterpret_cast<const __nv_bfloat16*>(sc + S.dz_lo[l]);
-        }
-        g.a.dlogits = io.head.dlogits;
-        g.a.dvalue = io.head.dvalue;
-        g.a.grads = grads;
-        g.a.B = B;
-        g.a.F = F;
-        g.traj = traj;
-        g.coefs = coefs;
-        g.logits = io.head.logits;
-        g.stats = stats;
-        g.acc = acc;
-        g.sc_stride = (long long)S.total;
-        g.illegal_stat = illegal_stat;
-        g.n_gram = gram_blocks(B, 1024);
-        launch_pdl(k_bias_grad_grouped, dim3(4 * (kHidden / 64) + 1 + (illegal_stat ? 1 : 0), (unsigned)K), dim3(1024), 0, s, g);
-    }
-    return check_launch(what);
+    auto ppo_heads = [](cudaStream_t st, const TrainHeadIO& head, const void* ctx) -> int32_t {
+        PpoGroupIO io = *static_cast<const PpoGroupIO*>(ctx);
+        io.head = head;
+        return launch_ppo_loss_grouped(st, io);
+    };
+    const TrainGroup group{p->n_learners, io.traj, io.coefs, io.stats, (p->flags & BRL_PPO_ILLEGAL_STAT) != 0};
+    TrainMinibatch t{};
+    t.obs_flags = p->flags & (BRL_PPO_OBS_U8 | BRL_PPO_OBS_BF16);
+    t.batch = p->batch;
+    t.blob = static_cast<const unsigned char*>(b[2]);
+    t.scratch = static_cast<unsigned char*>(b[3]);
+    t.grads = static_cast<float*>(b[4]);
+    t.grad_sumsq = static_cast<double*>(b[6]) + 14;  // learner k's |grads|^2: f64 14 of its accumulator slice
+    t.zero = b[6];
+    t.zero_bytes = 16 * sizeof(double);
+    t.tune = p->reserved & ~8;  // the tile trace (tune bit 3) records one learner's launches
+    t.what = "brl_ppo_grad_grouped";
+    t.loss_head = ppo_heads;
+    t.ctx = &io;
+    t.group = &group;
+    return launch_train_minibatch((cudaStream_t)stream, t);
 }
 
 int32_t brl_mlp_adam_step_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -1191,20 +1129,12 @@ int32_t brl_mlp_adam_step_grouped(brl_stream_t stream, void** b, const void* opa
     if (K == 0) return BRL_OK;  // no learners: a no-op, its buffers may be NULL
     if (K > BRL_MAX_LEARNERS) return fail(BRL_E_OPAQUE, "brl_mlp_adam_step_grouped: at most %d learners", BRL_MAX_LEARNERS);
     static const char* names[] = {"params", "grads", "m", "v", "acc", "blob"};
-    for (int k = 0; k < 6; ++k) {
-        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_mlp_adam_step_grouped: buffer '%s' is NULL", names[k]);
-        if ((reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0) return fail(BRL_E_BUFFER, "brl_mlp_adam_step_grouped: buffer '%s' is not 16-byte aligned", names[k]);
-    }
+    int32_t rc = check_buffers("brl_mlp_adam_step_grouped", b, names, 6, 0, 0x3Fu);
+    if (rc != BRL_OK) return rc;
     const BrlAdamParams* p = static_cast<const BrlAdamParams*>(opaque);
     GroupedAdamArgs g{};
-    for (int64_t k = 0; k < K; ++k) {
-        if (p[k].n != (int64_t)flat_layout().total || p[k].step <= 0)
-            return fail(BRL_E_OPAQUE, "brl_mlp_adam_step_grouped: learner %lld: n must be brl_mlp_num_params() and step (1-based) > 0", (long long)k);
-        AdamLearner& l = g.l[k];
-        l.max_norm = p[k].max_grad_norm; l.lr = p[k].lr; l.b1 = p[k].beta1; l.b2 = p[k].beta2; l.eps = p[k].eps;
-        l.bc1 = 1.0f - powf(p[k].beta1, (float)p[k].step);  // as brl_mlp_adam_step
-        l.bc2 = 1.0f - powf(p[k].beta2, (float)p[k].step);
-    }
+    for (int64_t k = 0; k < K; ++k)
+        if ((rc = adam_scalars("brl_mlp_adam_step_grouped", (long long)k, p[k], g.l[k])) != BRL_OK) return rc;
     g.a.p = static_cast<float*>(b[0]);
     g.a.g = static_cast<const float*>(b[1]);
     g.a.m = static_cast<float*>(b[2]);
@@ -1302,44 +1232,67 @@ static int train_ops(OpSpec* fwd, OpSpec* bwd, unsigned char* sc, const unsigned
         add_wgrad(2);
         add_wgrad(1);
     }
+    // a grouped launch: learner k's operands lie k scratches (activations, dz) or blobs (weights) after learner 0's
+    for (OpSpec* o = fwd; o != fwd + 5; ++o) { o->a_stride = (long long)S.total; o->w_stride = (long long)T.total; }
+    for (int i = 0; i < nb; ++i) {
+        bwd[i].a_stride = (long long)S.total;
+        bwd[i].w_stride = bwd[i].epi == kEpiWgrad ? (long long)S.total : (long long)T.total;
+    }
     return nb;
 }
 
+// one fused launch of the GEMMs at the tile width `wide` selects, for one learner (grp = NULL) or a group
+static int32_t launch_gemms(bool wide, cudaStream_t s, const OpSpec* ops, int n_ops, int nmb, uint32_t* ready,
+                            unsigned long long* trace, const char* what, const GroupSpec* grp) {
+    if (grp) return wide ? launch_fused_ops<128, true>(s, ops, n_ops, nmb, ready, trace, what, grp)
+                         : launch_fused_ops<64, true>(s, ops, n_ops, nmb, ready, trace, what, grp);
+    return wide ? launch_fused_ops<128>(s, ops, n_ops, nmb, ready, trace, what) : launch_fused_ops<64>(s, ops, n_ops, nmb, ready, trace, what);
+}
+
 int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
-    const int B = (int)t.batch;
+    const TrainGroup* grp = t.group;
+    const int B = (int)t.batch, K = grp ? grp->K : 1;
     const FlatLayout F = flat_layout();
     const TrainScratch S = train_scratch(B);
     unsigned char* sc = t.scratch;
     float* grads = t.grads;
     auto bf = [&](size_t off) { return reinterpret_cast<__nv_bfloat16*>(sc + off); };
+    const int nmb = ready_blocks(B);
+    uint32_t* ready = reinterpret_cast<uint32_t*>(sc + (grp ? grouped_ready_offset(K, B) : S.ready));
     int32_t rc = BRL_OK;
 
     // 0. counters and accumulators first, so that nothing but kernels (launched with programmatic dependent launch) follows
-    if (cudaMemsetAsync(sc + S.ready, 0, ready_words(B) * sizeof(uint32_t), s) != cudaSuccess ||
-        (t.zero != nullptr && cudaMemsetAsync(t.zero, 0, t.zero_bytes, s) != cudaSuccess))
+    if (cudaMemsetAsync(ready, 0, K * ready_words(B) * sizeof(uint32_t), s) != cudaSuccess ||
+        (t.zero != nullptr && (grp ? cudaMemset2DAsync(t.zero, BRL_PPO_SCRATCH_BYTES, 0, t.zero_bytes, (size_t)K, s)
+                                   : cudaMemsetAsync(t.zero, 0, t.zero_bytes, s)) != cudaSuccess))
         return check_launch(t.what);
-    // 1. minibatch gather of the observation (src/update.py:194-199, cast of src/update.py:95)
+    // 1. minibatch gather of the observation (src/update.py:194-199, cast of src/update.py:95); a group's learner k reads
+    //    row k of the trajectory table
     {
         const unsigned grid = (unsigned)(((int64_t)B * (kObsDimM / 8) + 255) / 256);
         uint16_t* o = reinterpret_cast<uint16_t*>(sc + S.obs);
-        if (t.obs_flags & BRL_PPO_OBS_BF16) launch_pdl(k_gather_obs<__nv_bfloat16>, dim3(grid), dim3(256), 0, s, static_cast<const __nv_bfloat16*>(t.obs), t.index, (int64_t)B, o);
-        else if (t.obs_flags & BRL_PPO_OBS_U8) launch_pdl(k_gather_obs<uint8_t>, dim3(grid), dim3(256), 0, s, static_cast<const uint8_t*>(t.obs), t.index, (int64_t)B, o);
-        else launch_pdl(k_gather_obs<float>, dim3(grid), dim3(256), 0, s, static_cast<const float*>(t.obs), t.index, (int64_t)B, o);
+        auto gather = [&](auto type) {
+            using T = decltype(type);
+            if (grp) launch_pdl(k_gather_obs_grouped<T>, dim3(grid, (unsigned)K), dim3(256), 0, s, grp->traj, (int64_t)B, o, (long long)S.total);
+            else launch_pdl(k_gather_obs<T>, dim3(grid), dim3(256), 0, s, static_cast<const T*>(t.obs), t.index, (int64_t)B, o);
+        };
+        if (t.obs_flags & BRL_PPO_OBS_BF16) gather(__nv_bfloat16{});
+        else if (t.obs_flags & BRL_PPO_OBS_U8) gather(uint8_t{});
+        else gather(float{});
     }
+    // 2. forward GEMMs; a group's as one launch over all learners' tiles, described by learner 0's ops
     OpSpec fwd[5], bwd[kMaxOps];
     const int nb = train_ops(fwd, bwd, sc, t.blob, grads, t.grad_sumsq, B);
-    double* grad_sumsq = t.grad_sumsq;
-    const int nmb = ready_blocks(B);
-    uint32_t* ready = reinterpret_cast<uint32_t*>(sc + S.ready);
+    const GroupSpec gs{K, (long long)S.total, (long long)train_blob().total, (long long)param_stride(), BRL_PPO_SCRATCH_BYTES / (long long)sizeof(double)};
+    const GroupSpec* g = grp ? &gs : nullptr;
     unsigned long long* trace = (t.tune & 8) ? reinterpret_cast<unsigned long long*>(sc + S.trace) : nullptr;  // tune bit 3
     // Tile widths, measured on B200 at B = 1024 (scripts/exp_train_trace.py): the forward is a chain of layers with one tile
     // per SM per layer, where 128 x 64 tiles win; the backward has two independent GEMMs per layer (dgrad, wgrad) to fill the
     // SMs, where 128 x 128 tiles move a third fewer operand bytes.  Tune bit 2 / bit 4 flip them.
     const bool wide_fwd = (t.tune & 4) != 0, wide_bwd = (t.tune & 16) == 0;
-    rc = wide_fwd ? launch_fused_ops<128>(s, fwd, 5, nmb, ready, trace, t.what) : launch_fused_ops<64>(s, fwd, 5, nmb, ready, trace, t.what);
-    if (rc != BRL_OK) return rc;
+    if ((rc = launch_gemms(wide_fwd, s, fwd, 5, nmb, ready, trace, t.what, g)) != BRL_OK) return rc;
     if ((rc = check_launch(t.what)) != BRL_OK) return rc;
-    // 3. the caller's loss head (and its backward into d loss / d (logits, value))
+    // 3. the caller's loss head (and its backward into d loss / d (logits, value)), given learner 0's buffers
     TrainHeadIO io{};
     io.logits = reinterpret_cast<const float*>(sc + S.logits);
     io.value = reinterpret_cast<const float*>(sc + S.value);
@@ -1350,16 +1303,29 @@ int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
     if ((rc = t.loss_head(s, io, t.ctx)) != BRL_OK) return rc;
     if (grads == nullptr) return BRL_OK;
     // 4. backward GEMMs
-    rc = wide_bwd ? launch_fused_ops<128>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr, t.what)
-                  : launch_fused_ops<64>(s, bwd, nb, nmb, ready + (size_t)kMaxOps * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr, t.what);
+    rc = launch_gemms(wide_bwd, s, bwd, nb, nmb, ready + (size_t)kMaxOps * K * (nmb + 1), trace ? trace + (size_t)kTraceTiles * 8 : nullptr,
+                      t.what, g);
     if (rc != BRL_OK) return rc;
-    // 5. bias gradients
-    {
-        BiasArgs a{};
-        for (int l = 0; l < 4; ++l) { a.hi[l] = bf(S.dz_hi[l]); a.lo[l] = bf(S.dz_lo[l]); }
-        a.dlogits = io.dlogits;
-        a.dvalue = io.dvalue;
-        a.grads = grads; a.sumsq = grad_sumsq; a.B = B; a.F = F;
+    // 5. bias gradients (and the deferred illegal-action statistic)
+    BiasArgs a{};
+    for (int l = 0; l < 4; ++l) { a.hi[l] = bf(S.dz_hi[l]); a.lo[l] = bf(S.dz_lo[l]); }
+    a.dlogits = io.dlogits;
+    a.dvalue = io.dvalue;
+    a.grads = grads; a.B = B; a.F = F;
+    if (grp) {
+        GroupedBiasArgs ga{};
+        ga.a = a;
+        ga.traj = grp->traj;
+        ga.coefs = grp->coefs;
+        ga.logits = io.logits;
+        ga.stats = grp->stats;
+        ga.acc = static_cast<unsigned char*>(t.zero);
+        ga.sc_stride = (long long)S.total;
+        ga.illegal_stat = grp->illegal_stat;
+        ga.n_gram = gram_blocks(B, 1024);
+        launch_pdl(k_bias_grad_grouped, dim3(4 * (kHidden / 64) + 1 + (grp->illegal_stat ? 1 : 0), (unsigned)K), dim3(1024), 0, s, ga);
+    } else {
+        a.sumsq = t.grad_sumsq;
         a.n_gram = t.gram ? t.n_gram : 0;
         if (a.n_gram) a.gram = *t.gram;
         launch_pdl(k_bias_grad, dim3(4 * (kHidden / 64) + 1 + (a.n_gram ? 1 : 0)), dim3(1024), 0, s, a);

@@ -432,13 +432,36 @@ brl::GramArgs brl::gram_args(void** b, const BrlPpoParams* p, float* stat) {
                         p->batch, static_cast<unsigned char*>(b[12]), stat);
 }
 
+// The loss head's launches, for one learner (Args = PpoArgs, a = g) or K (PpoGroupArgs, a = g.a, one grid row per learner):
+// `flags` decoded into `a`, then the advantage prepass (reward scaling), the Gram kernel (none when `gram` is NULL) and
+// the loss kernel.
+template <class Args, class GA>
+static int32_t launch_ppo_chain(cudaStream_t s, const Args& g, PpoArgs& a, int32_t flags, unsigned K, void (*gram)(GA), const GA& ga,
+                                const char* what) {
+    a.value_clipping = (flags & BRL_PPO_VALUE_CLIPPING) != 0;
+    a.reward_scaling = (flags & BRL_PPO_REWARD_SCALING) != 0;
+    a.masked_policy = (flags & BRL_PPO_UNMASKED_POLICY) == 0;
+    unsigned grid = (unsigned)((a.B + 3) / 4);
+    if (grid > 148u * 8u) grid = 148u * 8u;
+    const int prepass = a.reward_scaling;
+    if (prepass) k_ppo_prepass<Args><<<dim3(grid > 32u ? 32u : grid, K), 128, 0, s>>>(g);
+    if (gram) {
+        const dim3 gram_grid((unsigned)brl::gram_blocks(a.B, 1024), K);
+        if (prepass) gram<<<gram_grid, 1024, 0, s>>>(ga);  // a plain launch may not be followed by a PDL one that skips it
+        else launch_pdl(gram, gram_grid, dim3(1024), 0, s, ga);
+    }
+    launch_pdl(k_ppo_loss<Args>, dim3(grid, K), dim3(128), 0, s, g, prepass);
+    return check_launch(what);
+}
+
 int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* p, void* dz_hi, void* dz_lo, bool acc_zeroed,
                              bool defer_illegal) {
     if (p->batch <= 0) return fail(BRL_E_OPAQUE, "brl_ppo_loss: batch must be > 0");
     static const char* names[] = {"logits", "value", "index", "mask", "action", "old_log_prob", "old_value", "advantages",
                                   "targets", "dlogits", "dvalue", "stats", "scratch"};
-    for (int k = 0; k < 13; ++k)
-        if (b[k] == nullptr && k != 2) return fail(BRL_E_BUFFER, "brl_ppo_loss: buffer '%s' is NULL", names[k]);
+    const int32_t rc = check_buffers("brl_ppo_loss", b, names, 13, 1u << 2, 0);
+    if (rc != BRL_OK) return rc;
+    if (reinterpret_cast<uintptr_t>(b[12]) & 15u) return fail(BRL_E_BUFFER, "brl_ppo_loss: scratch is not 16-byte aligned");
     PpoArgs a{};
     a.logits = static_cast<const float*>(b[0]);
     a.value = static_cast<const float*>(b[1]);
@@ -453,7 +476,6 @@ int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* 
     a.dvalue = static_cast<float*>(b[10]);
     a.stats = static_cast<float*>(b[11]);
     a.acc = static_cast<double*>(b[12]);
-    if (reinterpret_cast<uintptr_t>(b[12]) & 15u) return fail(BRL_E_BUFFER, "brl_ppo_loss: scratch is not 16-byte aligned");
     a.spec = reinterpret_cast<double*>(static_cast<unsigned char*>(b[12]) + 128);
     a.gram_part = reinterpret_cast<float*>(static_cast<unsigned char*>(b[12]) + 512);
     a.dz_hi = static_cast<unsigned short*>(dz_hi);
@@ -463,26 +485,13 @@ int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* 
     a.ent_coef = p->ent_coef;
     a.vf_coef = p->vf_coef;
     a.ill_coef = p->illegal_l2_coef;
-    a.value_clipping = (p->flags & BRL_PPO_VALUE_CLIPPING) != 0;
-    a.reward_scaling = (p->flags & BRL_PPO_REWARD_SCALING) != 0;
-    a.masked_policy = (p->flags & BRL_PPO_UNMASKED_POLICY) == 0;
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!acc_zeroed && cudaMemsetAsync(a.acc, 0, 16 * sizeof(double), s) != cudaSuccess) return check_launch("brl_ppo_loss");
-    unsigned grid = (unsigned)((a.B + 3) / 4);
-    if (grid > 148u * 8u) grid = 148u * 8u;
-    const int prepass = a.reward_scaling;
-    if (prepass) k_ppo_prepass<PpoArgs><<<grid > 32u ? 32u : grid, 128, 0, s>>>(a);
     a.defer_illegal = defer_illegal && a.ill_coef == 0.0f;
     a.skip_illegal = a.defer_illegal && !(p->flags & BRL_PPO_ILLEGAL_STAT);
-    if (!a.skip_illegal) {
-        const GramArgs g = brl::gram_args(b, p, nullptr);
-        const unsigned gram_blocks = (unsigned)brl::gram_blocks(a.B, 1024);
-        auto kern = a.defer_illegal ? k_ppo_gram_partial : k_ppo_illegal_gram;
-        if (prepass) kern<<<gram_blocks, 1024, 0, s>>>(g);  // a plain launch may not be followed by a PDL one that skips it
-        else launch_pdl(kern, dim3(gram_blocks), dim3(1024), 0, s, g);
-    }
-    launch_pdl(k_ppo_loss<PpoArgs>, dim3(grid), dim3(128), 0, s, a, prepass);
-    return check_launch("brl_ppo_loss");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (!acc_zeroed && cudaMemsetAsync(a.acc, 0, 16 * sizeof(double), s) != cudaSuccess) return check_launch("brl_ppo_loss");
+    const GramArgs g = a.skip_illegal ? GramArgs{} : brl::gram_args(b, p, nullptr);
+    void (*gram)(GramArgs) = a.skip_illegal ? nullptr : a.defer_illegal ? k_ppo_gram_partial : k_ppo_illegal_gram;
+    return launch_ppo_chain(s, a, a, p->flags, 1u, gram, g, "brl_ppo_loss");
 }
 
 extern "C" {
@@ -496,8 +505,8 @@ static int32_t adam_impl(brl_stream_t stream, void** b, const void* opaque, size
         return fail(BRL_E_OPAQUE, "brl_adam_clip: opaque must be one BrlAdamParams (%zu bytes), got %zu", sizeof(BrlAdamParams), len);
     const BrlAdamParams* p = static_cast<const BrlAdamParams*>(opaque);
     static const char* names[] = {"params", "grads", "m", "v", "scratch"};
-    for (int k = 0; k < 5; ++k)
-        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "brl_adam_clip: buffer '%s' is NULL", names[k]);
+    const int32_t rc = check_buffers("brl_adam_clip", b, names, 5, 0, 0);
+    if (rc != BRL_OK) return rc;
     if (p->n <= 0 || p->step <= 0) return fail(BRL_E_OPAQUE, "brl_adam_clip: n and step (1-based) must be > 0");
     cudaStream_t s = (cudaStream_t)stream;
     double* sumsq = static_cast<double*>(b[4]);
@@ -563,23 +572,11 @@ int32_t brl::launch_ppo_loss_grouped(cudaStream_t s, const PpoGroupIO& io) {
     a.stats = io.stats;
     a.acc = reinterpret_cast<double*>(io.acc);
     a.B = io.batch;
-    a.value_clipping = (io.flags & BRL_PPO_VALUE_CLIPPING) != 0;
-    a.reward_scaling = (io.flags & BRL_PPO_REWARD_SCALING) != 0;
-    a.masked_policy = (io.flags & BRL_PPO_UNMASKED_POLICY) == 0;
     g.traj = io.traj;
     g.coefs = io.coefs;
     g.sc_stride = io.sc_stride;
     g.acc_stride = BRL_PPO_SCRATCH_BYTES;
     g.illegal_stat = (io.flags & BRL_PPO_ILLEGAL_STAT) != 0;
-    const unsigned K = (unsigned)io.K;
-    // the grids of launch_ppo_loss, one row per learner
-    unsigned grid = (unsigned)((a.B + 3) / 4);
-    if (grid > 148u * 8u) grid = 148u * 8u;
-    const int prepass = a.reward_scaling;
-    if (prepass) k_ppo_prepass<PpoGroupArgs><<<dim3(grid > 32u ? 32u : grid, K), 128, 0, s>>>(g);
-    const dim3 gram_grid((unsigned)brl::gram_blocks(a.B, 1024), K);
-    if (prepass) k_ppo_gram_grouped<<<gram_grid, 1024, 0, s>>>(g);  // a plain launch may not be followed by a PDL one that skips it
-    else launch_pdl(k_ppo_gram_grouped, gram_grid, dim3(1024), 0, s, g);
-    launch_pdl(k_ppo_loss<PpoGroupArgs>, dim3(grid, K), dim3(128), 0, s, g, prepass);
-    return check_launch("brl_ppo_grad_grouped");
+    // the Gram kernel runs for every learner: each decides from its own coefficient whether it has work
+    return launch_ppo_chain(s, g, a, io.flags, (unsigned)io.K, k_ppo_gram_grouped, g, "brl_ppo_grad_grouped");
 }

@@ -195,14 +195,10 @@ static int32_t sl_minibatch(const char* what, cudaStream_t s, void** b, const vo
     if (p->batch == 0) return BRL_OK;
     static const char* grad_names[] = {"obs", "blob", "scratch", "mask", "label", "grads", "stats", "acc"};
     static const char* eval_names[] = {"obs", "blob", "scratch", "mask", "label", "stats", "acc"};
-    const int nbuf = backward ? 8 : 7;
-    const char* const* names = backward ? grad_names : eval_names;
-    for (int k = 0; k < nbuf; ++k) {
-        if (b[k] == nullptr) return fail(BRL_E_BUFFER, "%s: buffer '%s' is NULL", what, names[k]);
-        const bool aligned16 = k <= 2 || (backward && k == 5) || k == nbuf - 1;
-        if (aligned16 && (reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0)
-            return fail(BRL_E_BUFFER, "%s: buffer '%s' is not 16-byte aligned", what, names[k]);
-    }
+    // obs, blob, scratch, grads and acc 16-byte aligned
+    const int32_t rc = backward ? check_buffers(what, b, grad_names, 8, 0, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 5 | 1u << 7)
+                                : check_buffers(what, b, eval_names, 7, 0, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 6);
+    if (rc != BRL_OK) return rc;
     SlHead head{};
     head.mask = static_cast<const uint8_t*>(b[3]);
     head.label = static_cast<const int32_t*>(b[4]);

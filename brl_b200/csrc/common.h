@@ -94,6 +94,17 @@ struct TrainHeadIO {  // what the forward leaves for the loss head, and where th
     void* dz_hi;          // bf16 hi / lo [B, 64]: 38 logits, value, zeros (the head's dgrad / wgrad operand)
     void* dz_lo;
 };
+// K learners in the launches of one minibatch (brl_ppo_grad_grouped), learner 0's buffers in TrainMinibatch: learner k's
+// scratch lies k * train_scratch(batch).total bytes further, its blob k * brl_mlp_train_blob_bytes(), its grads
+// k * brl_mlp_param_stride() floats, its accumulators (`zero`, `grad_sumsq`) k * BRL_PPO_SCRATCH_BYTES bytes; the grouped
+// tile counters follow the K scratches.  `obs` and `index` are unused: they come from the trajectory table.
+struct TrainGroup {
+    int K;
+    const long long* traj;  // [K][8] (ops.ppo_trajectory_row): the gather reads obs and index, the Gram tail index and mask
+    const float* coefs;     // [K][4]: the Gram tail runs for a learner whose illegal_l2_coef (column 3) is 0
+    float* stats;           // [K][8]
+    bool illegal_stat;      // BRL_PPO_ILLEGAL_STAT
+};
 struct TrainMinibatch {
     const void* obs;             // [total, 480] f32, or u8 / bf16 with obs_flags BRL_PPO_OBS_U8 / BRL_PPO_OBS_BF16
     int32_t obs_flags;
@@ -111,6 +122,7 @@ struct TrainMinibatch {
     const char* what;            // op name for error messages
     int32_t (*loss_head)(cudaStream_t, const TrainHeadIO&, const void* ctx);
     const void* ctx;
+    const TrainGroup* group;     // NULL = one learner
 };
 int32_t launch_train_minibatch(cudaStream_t stream, const TrainMinibatch& t);
 
@@ -160,5 +172,16 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
         if ((reinterpret_cast<uintptr_t>(ptr) & 15u) != 0)                                \
             return brl::fail(BRL_E_BUFFER, "%s: buffer '%s' is not 16-byte aligned", __func__, name);    \
     } while (0)
+
+// An op's buffer checks, in buffer order: b[k] must not be NULL unless bit k of `nullable` is set, and must be 16-byte
+// aligned when bit k of `aligned16` is set.  `what` names the op in the message.
+inline int32_t check_buffers(const char* what, void* const* b, const char* const* names, int n, unsigned nullable, unsigned aligned16) {
+    for (int k = 0; k < n; ++k) {
+        if (b[k] == nullptr && !((nullable >> k) & 1u)) return fail(BRL_E_BUFFER, "%s: buffer '%s' is NULL", what, names[k]);
+        if (((aligned16 >> k) & 1u) && (reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0)
+            return fail(BRL_E_BUFFER, "%s: buffer '%s' is not 16-byte aligned", what, names[k]);
+    }
+    return BRL_OK;
+}
 
 }  // namespace brl

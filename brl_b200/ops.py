@@ -331,12 +331,26 @@ def ppo_scratch(device) -> torch.Tensor:
     return torch.zeros(_lib.PPO_SCRATCH_BYTES // 8, dtype=torch.float64, device=device)
 
 
+def _ppo_flags(op, *, value_clipping, reward_scaling, masked_policy, illegal_stat=False, obs_dtype=None) -> int:
+    """BrlPpoParams.flags of `op`; obs_dtype = the observations' dtype (None: the op reads none)"""
+    try:
+        oflag = {None: 0, torch.float32: 0, torch.uint8: _lib.PPO_OBS_U8, torch.bool: _lib.PPO_OBS_U8,
+                 torch.bfloat16: _lib.PPO_OBS_BF16}[obs_dtype]
+    except KeyError:
+        raise _lib.BrlError(f"{op}: observation dtype {obs_dtype} not supported") from None
+    return (_lib.PPO_VALUE_CLIPPING if value_clipping else 0) | (_lib.PPO_REWARD_SCALING if reward_scaling else 0) | \
+        (0 if masked_policy else _lib.PPO_UNMASKED_POLICY) | (_lib.PPO_ILLEGAL_STAT if illegal_stat else 0) | oflag
+
+
+def _adam_params(n, step, lr, beta1, beta2, eps, max_grad_norm):
+    return _lib.BrlAdamParams(int(n), int(step), float(lr), float(beta1), float(beta2), float(eps), float(max_grad_norm))
+
+
 def ppo_loss(logits, value, index, mask, action, old_log_prob, old_value, adv, targets, dlogits, dvalue, stats, scratch,
              *, clip_eps, ent_coef, vf_coef, illegal_l2_coef=0.0, value_clipping=True, reward_scaling=False,
              masked_policy=True) -> None:
     """_loss_fn of src/update.py:91-162 + its gradient w.r.t. (logits, value) for one minibatch."""
-    flags = (_lib.PPO_VALUE_CLIPPING if value_clipping else 0) | (_lib.PPO_REWARD_SCALING if reward_scaling else 0) | \
-            (0 if masked_policy else _lib.PPO_UNMASKED_POLICY)
+    flags = _ppo_flags("ppo_loss", value_clipping=value_clipping, reward_scaling=reward_scaling, masked_policy=masked_policy)
     p = _lib.BrlPpoParams(int(logits.shape[0]), int(action.numel()), float(clip_eps), float(ent_coef), float(vf_coef),
                           float(illegal_l2_coef), flags, 0)
     _call("brl_ppo_loss", [_ptr(logits), _ptr(value), _ptr(index), _ptr(mask), _ptr(action), _ptr(old_log_prob),
@@ -348,8 +362,7 @@ def adam_clip(params, grads, m, v, scratch, *, step: int, lr: float, beta1=0.9, 
               max_grad_norm=0.0, sumsq: Optional[torch.Tensor] = None) -> None:
     """optax.chain(clip_by_global_norm, adam) on flat fp32 buffers, in place (ppo.py:195-211).  `sumsq` (f64[1], e.g.
     `acc[14:15]` after `ppo_grad`): the gradient's sum of squares is already known, skip the pass that forms it."""
-    p = _lib.BrlAdamParams(int(params.numel()), int(step), float(lr), float(beta1), float(beta2), float(eps),
-                           float(max_grad_norm))
+    p = _adam_params(params.numel(), step, lr, beta1, beta2, eps, max_grad_norm)
     if sumsq is not None:
         if sumsq.dtype != torch.float64:
             raise _lib.BrlError("adam_clip: sumsq must be float64")
@@ -380,8 +393,7 @@ def mlp_adam_step(params, grads, m, v, sumsq, blob, *, step: int, lr: float, bet
     the same pass (ppo.py:195-211, src/update.py:168-169).  `sumsq`: f64[1] = `acc[14:15]` after `ppo_grad`."""
     if sumsq.dtype != torch.float64:
         raise _lib.BrlError("mlp_adam_step: sumsq must be float64")
-    p = _lib.BrlAdamParams(int(params.numel()), int(step), float(lr), float(beta1), float(beta2), float(eps),
-                           float(max_grad_norm))
+    p = _adam_params(params.numel(), step, lr, beta1, beta2, eps, max_grad_norm)
     _call("brl_mlp_adam_step", [_ptr(params), _ptr(grads), _ptr(m), _ptr(v), _ptr(sumsq), _ptr(blob)], p)
 
 
@@ -399,16 +411,12 @@ def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, a
     B = int(index.shape[0]) if index is not None else int(obs.shape[0])
     if obs.dtype == torch.bool:
         obs = obs.view(torch.uint8)
-    try:
-        oflag = {torch.float32: 0, torch.uint8: _lib.PPO_OBS_U8, torch.bfloat16: _lib.PPO_OBS_BF16}[obs.dtype]
-    except KeyError:
-        raise _lib.BrlError(f"ppo_grad: observation dtype {obs.dtype} not supported") from None
+    flags = _ppo_flags("ppo_grad", value_clipping=value_clipping, reward_scaling=reward_scaling, masked_policy=masked_policy,
+                       illegal_stat=illegal_stat, obs_dtype=obs.dtype)
     if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
         raise _lib.BrlError("ppo_grad: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
     if grads.dtype != torch.float32 or grads.numel() != L.brl_mlp_num_params():
         raise _lib.BrlError("ppo_grad: grads must be the flat fp32 gradient buffer")
-    flags = (_lib.PPO_VALUE_CLIPPING if value_clipping else 0) | (_lib.PPO_REWARD_SCALING if reward_scaling else 0) | \
-            (0 if masked_policy else _lib.PPO_UNMASKED_POLICY) | (_lib.PPO_ILLEGAL_STAT if illegal_stat else 0) | oflag
     p = _lib.BrlPpoParams(B, int(action.numel()), float(clip_eps), float(ent_coef), float(vf_coef), float(illegal_l2_coef),
                           flags, int(tune))
     _call("brl_ppo_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(index), _ptr(mask), _ptr(action), _ptr(old_log_prob),
@@ -456,13 +464,8 @@ def ppo_grad_grouped(traj, coefs, blob, scratch, grads, stats, acc, *, batch: in
             acc.dtype != torch.float64 or acc.numel() != K * (_lib.PPO_SCRATCH_BYTES // 8):
         raise _lib.BrlError("ppo_grad_grouped: blob must be uint8[K, mlp_train_blob_bytes], acc float64[K, PPO_SCRATCH_BYTES / 8], "
                             "scratch ppo_grad_grouped_scratch_bytes(K, batch)")
-    try:
-        oflag = {torch.float32: 0, torch.uint8: _lib.PPO_OBS_U8, torch.bool: _lib.PPO_OBS_U8,
-                 torch.bfloat16: _lib.PPO_OBS_BF16}[obs_dtype]
-    except KeyError:
-        raise _lib.BrlError(f"ppo_grad_grouped: observation dtype {obs_dtype} not supported") from None
-    flags = (_lib.PPO_VALUE_CLIPPING if value_clipping else 0) | (_lib.PPO_REWARD_SCALING if reward_scaling else 0) | \
-            (0 if masked_policy else _lib.PPO_UNMASKED_POLICY) | (_lib.PPO_ILLEGAL_STAT if illegal_stat else 0) | oflag
+    flags = _ppo_flags("ppo_grad_grouped", value_clipping=value_clipping, reward_scaling=reward_scaling, masked_policy=masked_policy,
+                       illegal_stat=illegal_stat, obs_dtype=obs_dtype)
     p = _lib.BrlPpoGroupedParams(int(batch), K, flags, int(tune), 0)
     _call("brl_ppo_grad_grouped", [_ptr(traj), _ptr(coefs), _ptr(blob), _ptr(scratch), _ptr(grads), _ptr(stats), _ptr(acc)], p)
 
@@ -489,8 +492,7 @@ def mlp_adam_step_grouped(params, grads, m, v, acc, blob, *, steps, lrs, max_gra
     def per(x):
         return list(x) if isinstance(x, (list, tuple)) else [x] * K
     b1, b2, ep = per(beta1), per(beta2), per(eps)
-    p = (_lib.BrlAdamParams * K)(*[_lib.BrlAdamParams(n, int(steps[k]), float(lrs[k]), float(b1[k]), float(b2[k]), float(ep[k]),
-                                                       float(max_grad_norms[k])) for k in range(K)])
+    p = (_lib.BrlAdamParams * K)(*[_adam_params(n, steps[k], lrs[k], b1[k], b2[k], ep[k], max_grad_norms[k]) for k in range(K)])
     _call("brl_mlp_adam_step_grouped", [_ptr(params), _ptr(grads), _ptr(m), _ptr(v), _ptr(acc), _ptr(blob)], p)
 
 

@@ -19,14 +19,13 @@ from .optim import OptState, flatten_params, update_mlp_grouped_
 _STAT_NAMES = ("total_loss", "value_loss", "loss_actor", "entropy", "approx_kl", "clipflacs", "illegal_action_loss")
 
 
-def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None):
-    """`permutation_fn(rng, batch_size) -> int64/32 tensor` replaces jax.random.permutation
-    (src/update.py:193); default: torch.randperm seeded by the key (tests inject a fixed one)."""
-    masked = bool(config["actor_illegal_action_mask"])
-    cfg = dict(clip_eps=config["clip_eps"], ent_coef=config["ent_coef"], vf_coef=config["vf_coef"],
-               illegal_l2_coef=config.get("illegal_action_l2norm_coef", 0.0),
-               value_clipping=bool(config.get("value_clipping", True)),
-               reward_scaling=bool(config.get("reward_scaling", False)), masked_policy=masked)
+def _loss_settings(config, actor_forward_pass, who):
+    """One learner's loss settings: (ppo_grad's flag keywords, its coefficient row [clip_eps, ent_coef, vf_coef,
+    illegal_l2_coef], the illegal_action_loss statistic mode, brl_train_tune)."""
+    flags = dict(value_clipping=bool(config.get("value_clipping", True)), reward_scaling=bool(config.get("reward_scaling", False)),
+                 masked_policy=bool(config["actor_illegal_action_mask"]))
+    coefs = [float(config["clip_eps"]), float(config["ent_coef"]), float(config["vf_coef"]),
+             float(config.get("illegal_action_l2norm_coef", 0.0))]
     # illegal_action_loss = ||probs * ~mask||_2 / 2 is the SPECTRAL norm of the [minibatch, 38] matrix (src/update.py:141-142): a
     # 38 x 38 eigen-problem per minibatch.  With the default illegal_action_l2norm_coef = 0 it is a logged statistic only,
     # and ppo.py logs just the LAST minibatch of the last epoch (ppo.py:505, `illegal_action_loss[-1][-1]`).  "last" (default)
@@ -37,31 +36,53 @@ def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None)
     if stat_mode not in ("last", "all"):
         raise ValueError("illegal_action_loss_stat must be 'last' or 'all'")
     if getattr(actor_forward_pass, "precision", None) not in ("tc", "tc-bf16"):
-        raise TypeError("make_update_step needs a brl_b200.models.ForwardPass (tensor-core ReLU net); there is no library "
-                        "back end on the product path")
-    tune = int(config.get("brl_train_tune", 0))
+        raise TypeError(f"{who} needs a brl_b200.models.ForwardPass (tensor-core ReLU net); there is no library back end on the "
+                        "product path")
+    return flags, coefs, stat_mode, int(config.get("brl_train_tune", 0))
 
-    def default_permutation(rng, batch_size, device):
-        g = torch.Generator(device="cpu").manual_seed(rng & 0x7FFFFFFFFFFFFFFF)
-        return torch.randperm(batch_size, generator=g).to(device=device, dtype=torch.int32)
+
+def _flat_rollout(traj_batch, advantages, targets, batch_size):
+    """The ppo_grad buffers of one learner's rollout, flat over (step, env) (src/update.py:195-197): obs, mask, action,
+    old_log_prob, old_value, advantages, targets."""
+    T, n = advantages.shape
+    assert batch_size == T * n, "batch size must be equal to number of steps * number of envs"  # src/update.py:189-192
+    obs = traj_batch.obs.reshape(batch_size, -1)
+    if obs.dtype == torch.bool:
+        obs = obs.view(torch.uint8)
+    return (obs.contiguous(), traj_batch.legal_action_mask.reshape(batch_size, -1).view(torch.uint8).contiguous(),
+            traj_batch.action.reshape(batch_size).contiguous(), traj_batch.log_prob.reshape(batch_size).contiguous(),
+            traj_batch.value.reshape(batch_size).contiguous(), advantages.reshape(batch_size).contiguous(),
+            targets.reshape(batch_size).contiguous())
+
+
+def _permutation(permutation_fn, rng, batch_size, device):
+    """One epoch's minibatch order (src/update.py:193): `permutation_fn`, or torch.randperm seeded by the key."""
+    if permutation_fn is not None:
+        perm = permutation_fn(rng, batch_size)
+    else:
+        perm = torch.randperm(batch_size, generator=torch.Generator(device="cpu").manual_seed(rng & 0x7FFFFFFFFFFFFFFF))
+    return perm.to(device=device, dtype=torch.int32).contiguous()
+
+
+def _loss_info(stats):
+    """loss_info from stats[update_epochs, num_minibatches, 8]: (total_loss, (value_loss, loss_actor, entropy, approx_kl,
+    clipflacs, illegal_action_loss)), each [update_epochs, num_minibatches] (src/update.py:170-173, 226-229; read at
+    ppo.py:487-506)"""
+    cols = [stats[:, :, i] for i in range(7)]
+    return cols[0], tuple(cols[1:])
+
+
+def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None):
+    """`permutation_fn(rng, batch_size) -> int64/32 tensor` replaces jax.random.permutation
+    (src/update.py:193); default: torch.randperm seeded by the key (tests inject a fixed one)."""
+    flags, coefs, stat_mode, tune = _loss_settings(config, actor_forward_pass, "make_update_step")
+    cfg = dict(zip(("clip_eps", "ent_coef", "vf_coef", "illegal_l2_coef"), coefs), **flags)
 
     def update_step(runner_state, traj_batch, advantages, targets):
         params, opt_state, env_state, last_obs, terminated_count, rng = runner_state
         dev = advantages.device
         nmb, mbs = int(config["num_minibatches"]), int(config["minibatch_size"])
-        batch_size = nmb * mbs
-        T, n = advantages.shape
-        assert batch_size == T * n, "batch size must be equal to number of steps * number of envs"  # src/update.py:189-192
-        # flat views of the rollout (src/update.py:195-197)
-        obs = traj_batch.obs.reshape(batch_size, -1)
-        mask = traj_batch.legal_action_mask.reshape(batch_size, -1).view(torch.uint8).contiguous()
-        action = traj_batch.action.reshape(batch_size).contiguous()
-        old_lp = traj_batch.log_prob.reshape(batch_size).contiguous()
-        old_v = traj_batch.value.reshape(batch_size).contiguous()
-        adv, tgt = advantages.reshape(batch_size).contiguous(), targets.reshape(batch_size).contiguous()
-        if obs.dtype == torch.bool:
-            obs = obs.view(torch.uint8)
-        obs = obs.contiguous()
+        obs, mask, action, old_lp, old_v, adv, tgt = _flat_rollout(traj_batch, advantages, targets, nmb * mbs)
 
         flat_p, new_params = flatten_params(params)
         if opt_state is None:
@@ -70,29 +91,18 @@ def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None)
         n_epochs = int(config["update_epochs"])
         stats_all = torch.zeros((n_epochs, nmb, 8), dtype=torch.float32, device=dev)
         acc = ops.ppo_scratch(dev)
-
-        def permutation(_rng):
-            return (permutation_fn(_rng, batch_size) if permutation_fn is not None
-                    else default_permutation(_rng, batch_size, dev)).to(device=dev, dtype=torch.int32).contiguous()
-
-        def finish():
-            # loss_info: (total_loss, (value_loss, loss_actor, entropy, approx_kl, clipflacs, illegal_action_loss)),
-            # each [update_epochs, num_minibatches] (src/update.py:170-173, 226-229; read at ppo.py:487-506)
-            cols = [stats_all[:, :, i] for i in range(7)]
-            return (new_params, state, env_state, last_obs, terminated_count, rng), (cols[0], tuple(cols[1:]))
-
         blob = ops.mlp_pack_train(flat_p)
         scratch = ops.mlp_train_scratch(mbs, dev)
         flat_g = torch.empty_like(flat_p)
         for epoch in range(n_epochs):
             rng, _rng = brandom.split(rng)                                        # src/update.py:187
-            perm = permutation(_rng)
+            perm = _permutation(permutation_fn, _rng, nmb * mbs, dev)
             for mb in range(nmb):                                                  # src/update.py:207-209
                 ops.ppo_grad(obs, blob, scratch, perm[mb * mbs:(mb + 1) * mbs], mask, action, old_lp, old_v, adv, tgt,
                              flat_g, stats_all[epoch, mb], acc, tune=tune, illegal_stat=stat_mode == "all" or mb == nmb - 1,
                              **cfg)                                                # src/update.py:164-167
                 state = optimizer.update_mlp_(flat_p, flat_g, state, acc[14:15], blob)  # src/update.py:168-169
-        return finish()
+        return (new_params, state, env_state, last_obs, terminated_count, rng), _loss_info(stats_all)
 
     return update_step
 
@@ -129,23 +139,11 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
         raise ValueError("make_population_update_step needs one optimizer per config")
     if len(configs) > _lib.MAX_LEARNERS:
         raise ValueError(f"a population has at most {_lib.MAX_LEARNERS} learners")
+    settings = [_loss_settings(c, actor_forward_pass, "make_population_update_step") for c in configs]
+    flags, _, stat_mode, tune = settings[0]  # shared keys: equal for every learner
+    coef_rows = [coefs for _, coefs, _, _ in settings]
     c0 = configs[0]
-    masked = bool(c0["actor_illegal_action_mask"])
-    flags = dict(value_clipping=bool(c0.get("value_clipping", True)), reward_scaling=bool(c0.get("reward_scaling", False)),
-                 masked_policy=masked)
-    coef_rows = [[float(c["clip_eps"]), float(c["ent_coef"]), float(c["vf_coef"]), float(c.get("illegal_action_l2norm_coef", 0.0))]
-                 for c in configs]
-    stat_mode = c0.get("illegal_action_loss_stat", "last")
-    if stat_mode not in ("last", "all"):
-        raise ValueError("illegal_action_loss_stat must be 'last' or 'all'")
-    if getattr(actor_forward_pass, "precision", None) not in ("tc", "tc-bf16"):
-        raise TypeError("make_population_update_step needs a brl_b200.models.ForwardPass (tensor-core ReLU net)")
-    tune = int(c0.get("brl_train_tune", 0))
     K = len(configs)
-
-    def default_permutation(rng, batch_size, device):
-        g = torch.Generator(device="cpu").manual_seed(rng & 0x7FFFFFFFFFFFFFFF)
-        return torch.randperm(batch_size, generator=g).to(device=device, dtype=torch.int32)
 
     def update_step(runner_states, traj_batches, advantages, targets):
         if not (len(runner_states) == len(traj_batches) == len(advantages) == len(targets) == K):
@@ -154,21 +152,10 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
         nmb, mbs = int(c0["num_minibatches"]), int(c0["minibatch_size"])
         batch_size = nmb * mbs
         n_epochs = int(c0["update_epochs"])
-        flat = []  # per learner: the ppo_grad buffers of its flat rollout (src/update.py:195-197)
-        obs_dtype = None
-        for tb, adv, tgt in zip(traj_batches, advantages, targets):
-            T, n = adv.shape
-            assert batch_size == T * n, "batch size must be equal to number of steps * number of envs"
-            obs = tb.obs.reshape(batch_size, -1)
-            if obs.dtype == torch.bool:
-                obs = obs.view(torch.uint8)
-            if obs_dtype is not None and obs.dtype != obs_dtype:
-                raise ValueError("population learners must record observations of one dtype")
-            obs_dtype = obs.dtype
-            flat.append((obs.contiguous(), tb.legal_action_mask.reshape(batch_size, -1).view(torch.uint8).contiguous(),
-                         tb.action.reshape(batch_size).contiguous(), tb.log_prob.reshape(batch_size).contiguous(),
-                         tb.value.reshape(batch_size).contiguous(), adv.reshape(batch_size).contiguous(),
-                         tgt.reshape(batch_size).contiguous()))
+        flat = [_flat_rollout(tb, adv, tgt, batch_size) for tb, adv, tgt in zip(traj_batches, advantages, targets)]
+        obs_dtype = flat[0][0].dtype
+        if any(f[0].dtype != obs_dtype for f in flat):
+            raise ValueError("population learners must record observations of one dtype")
 
         n_params, blob_bytes = ops.mlp_num_params(), int(_lib.load().brl_mlp_train_blob_bytes())
         flat_p = torch.zeros((K, ops.mlp_param_stride()), dtype=torch.float32, device=dev)  # learner k: flat_p[k, :n_params]
@@ -194,15 +181,11 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
         scratch = torch.empty(ops.ppo_grad_grouped_scratch_bytes(K, mbs), dtype=torch.uint8, device=dev)
         coefs = torch.tensor(coef_rows, dtype=torch.float32).to(dev)
 
-        def permutation(_rng):
-            return (permutation_fn(_rng, batch_size) if permutation_fn is not None
-                    else default_permutation(_rng, batch_size, dev)).to(device=dev, dtype=torch.int32).contiguous()
-
         for epoch in range(n_epochs):
             perms = []
             for k in range(K):
                 rngs[k], _rng = brandom.split(rngs[k])                            # src/update.py:187
-                perms.append(permutation(_rng))
+                perms.append(_permutation(permutation_fn, _rng, batch_size, dev))
             # this epoch's trajectory tables, one [K, 8] per minibatch: the index column steps through each permutation
             base = torch.tensor([ops.ppo_trajectory_row(f[0], perms[k], *f[1:]) for k, f in enumerate(flat)], dtype=torch.int64)
             tables = base.repeat(nmb, 1, 1)
@@ -215,9 +198,8 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
 
         out = []
         for k in range(K):
-            cols = [stats_all[:, :, k, i] for i in range(7)]
             env_state, last_obs, terminated_count = rest[k]
-            out.append(((new_params[k], states[k], env_state, last_obs, terminated_count, rngs[k]), (cols[0], tuple(cols[1:]))))
+            out.append(((new_params[k], states[k], env_state, last_obs, terminated_count, rngs[k]), _loss_info(stats_all[:, :, k])))
         return out
 
     return update_step

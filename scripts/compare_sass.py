@@ -8,9 +8,8 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES records the population-training change: k_train_fused gained a GROUPED flag (the solo kernels are GROUPED = false)
-and k_ppo_prepass / k_ppo_loss became templates over their argument type (the solo kernels take PpoArgs),
-and ADDED lists the grouped kernels it adds.  Replace both tables for another change."""
+RENAMES and ADDED record the PPO update's host-side refactor, which changes no device code: both are empty.  Replace both
+tables for another change."""
 import argparse
 import os
 import re
@@ -18,18 +17,8 @@ import subprocess
 import sys
 from collections import OrderedDict
 
-RENAMES = [  # demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-    (r"^brl::k_train_fused<\(int\)(\d+)>$", r"brl::k_train_fused<(int)\1, (bool)0>"),
-    (r"^brl::k_ppo_(prepass|loss)$", r"brl::k_ppo_\1<brl::PpoArgs>"),
-]
-ADDED = [  # kernels the change adds on purpose: reported, not counted as unexpected
-    r"^brl::k_train_fused<\(int\)\d+, \(bool\)1>$",
-    r"^brl::k_gather_obs_grouped<.*>$",
-    r"^brl::k_bias_grad_grouped$",
-    r"^brl::k_adam_pack_grouped$",
-    r"^brl::k_ppo_(prepass|loss)<brl::PpoGroupArgs>$",
-    r"^brl::k_ppo_gram_grouped$",
-]
+RENAMES = []  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
+ADDED = []  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):
