@@ -20,13 +20,15 @@ import numpy as np
 import torch
 
 from . import deals as _deals
+from . import pbt as _pbt
 from . import random as brandom
 from .env import BridgeBidding
 from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_pfsp_probe,
                          make_device_simple_evaluate, make_evaluate_log)
 from .gae import make_calc_gae
 from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
-from .optim import make_optimizer
+from .optim import OptState, make_optimizer
+from .pbt import default_pbt_config  # noqa: F401 -- ppo.default_pbt_config(): the options of train_population's `pbt`
 from .roll_out import make_roll_out
 from .update import check_population_configs, make_population_update_step, make_update_step
 from .zoo import ModelZoo, device_zoo_fits
@@ -125,7 +127,7 @@ class Learner:
             params = load_params(config["initial_model_path"], dev)                                   # ppo.py:246-248
 
         rng, self.eval_rng = brandom.split(rng)
-        eval_env = BridgeBidding(table=eval_table, device=dev)
+        self.eval_env = eval_env = BridgeBidding(table=eval_table, device=dev)
         if eval_opp_params is None:
             eval_opp_params = (load_params(config["eval_opp_model_path"], dev) if config["eval_opp_model_path"]
                                else init_params(12345, dev))
@@ -172,6 +174,7 @@ class Learner:
         if config["save_model"]:
             os.makedirs(self.save_dir, exist_ok=True)
         self.logs = []
+        self.pbt_lineage = None  # train_population with PBT: [iteration, parent, {key: value}] per PBT step
 
     def zoo_model(self, k: int):
         if self.device_zoo:
@@ -230,8 +233,9 @@ class Learner:
         self.runner_state = runner_state
         return traj_batch, advantages, targets
 
-    def finish_iteration(self, i: int, runner_state, loss_info, t_update: float) -> dict:
-        """Iteration i after the update (ppo.py:479-549): the strength probe, the log, the table rotation."""
+    def finish_iteration(self, i: int, runner_state, loss_info, t_update: float, emit: bool = True) -> dict:
+        """Iteration i after the update (ppo.py:479-549): the strength probe, the log, the table rotation.  `emit=False`
+        leaves the log_fn call to the caller (`emit`), which adds entries to the log first."""
         config, dev = self.config, self.dev
         self.runner_state = runner_state
         (imp_opp_after, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, self.eval_rng)
@@ -250,8 +254,8 @@ class Learner:
         }
         log.update(self.eval_log)
         self.logs.append(log)
-        if self.log_fn is not None:
-            self.log_fn(log)
+        if emit:
+            self.emit(log)
         if (board_num - self.board_count) // config["hash_size"] >= 1:                            # ppo.py:525-549
             self.hash_index += 1
             self.board_count = board_num
@@ -266,6 +270,28 @@ class Learner:
             log["table"] = int(k)
         return log
 
+    def emit(self, log: dict) -> None:
+        if self.log_fn is not None:
+            self.log_fn(log)
+
+    def adopt(self, src: "Learner", values: dict) -> None:
+        """PBT's exploit and explore: take `src`'s parameters and Adam state (device copies into this learner's own
+        buffers, on the current stream) and set the config `values`, rebuilding the optimizer that captured them.  The
+        update step holds the loss coefficients and optimizers and is the caller's to rebuild.  Env state, rollout key,
+        table rotation, zoo and save directory stay this learner's; a self-play opponent becomes the new parameters."""
+        params, opt_state = self.runner_state[:2]
+        src_params, src_state = src.runner_state[:2]
+        for name in LAYERS:
+            for k in ("w", "b"):
+                params[name][k].copy_(src_params[name][k])
+        opt_state.mu.copy_(src_state.mu)
+        opt_state.nu.copy_(src_state.nu)
+        self.runner_state = (params, OptState(src_state.count, opt_state.mu, opt_state.nu)) + tuple(self.runner_state[2:])
+        self.config.update(values)
+        self.optimizer = make_optimizer(self.config)
+        if self.config["self_play"]:
+            self.opp_params = params
+
     def finish(self):
         """The final save (ppo.py:550-569); -> (runner_state, logs) as `train` returns them."""
         config = self.config
@@ -274,6 +300,8 @@ class Learner:
             with open(os.path.join(self.save_dir, f"opt_state-{config['num_updates']:08}.pkl"), "wb") as fh:
                 st = self.runner_state[1]
                 pickle.dump({"count": st.count, "mu": st.mu.cpu().numpy(), "nu": st.nu.cpu().numpy()}, fh)
+            if self.pbt_lineage is not None:
+                _pbt.write_lineage(os.path.join(self.save_dir, "pbt_lineage.json"), self.pbt_lineage)
         return self.runner_state, self.logs
 
 
@@ -296,22 +324,37 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
 
 def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optional[Sequence] = None, eval_table=None,
                      device="cuda", log_fns: Optional[Sequence[Optional[Callable[[dict], None]]]] = None,
-                     eval_opp_params=None, np_rngs: Optional[Sequence[Optional[np.random.Generator]]] = None):
+                     eval_opp_params=None, np_rngs: Optional[Sequence[Optional[np.random.Generator]]] = None,
+                     pbt: Optional[dict] = None):
     """`train` for K learners on one GPU.  Each learner runs its own control plane (evaluations, FSP / PFSP opponents and
     zoo, rollout, GAE, logging, table rotation) in turn, and the K updates of an iteration run as one grouped update step
     (update.make_population_update_step), so that the learners' GEMM tiles share the device.  configs[k] and rngs[k] give
     learner k exactly the run `train(configs[k], rngs[k], ...)` gives; the keys of update.POPULATION_SHARED_KEYS must be
-    equal across learners (ValueError naming the first that is not).  -> [(runner_state, logs)] per learner."""
+    equal across learners (ValueError naming the first that is not).  -> [(runner_state, logs)] per learner.
+
+    `pbt`: population-based training (brl_b200/pbt.py), a dict of options over default_pbt_config(): `interval`
+    (iterations between rankings; 10), `metric` ("league": each learner's mean IMP in a round robin of the K current nets
+    on `league_boards` (100) boards of the eval table; "score": its latest train/score), `quantile` (0.25: n = max(1,
+    floor(quantile * K)) of the lowest learners each copy the parameters and Adam state of one of the n highest),
+    `perturb_keys` (("lr", "ent_coef"): the winner's values the loser takes, each multiplied by a factor drawn from
+    `perturb_factors`, (0.8, 1.25)) and `seed` (the population's generator of those draws).  Rankings run at iterations
+    i > 0 with i % interval == 0, after every learner's finish_iteration; that iteration's logs gain pbt/fitness,
+    pbt/rank (0 = fittest), pbt/parent (the learner copied, or -1) and pbt/<key> for each perturbed key before log_fns
+    see them, and with save_model each learner's save directory gets a pbt_lineage.json.  ValueError (before any device work) for K < 2, a quantile outside (0, 0.5], a perturbed key that
+    default_config() does not know or that the population shares, and the other bad options pbt.check_pbt_config lists.
+    None (the default) trains the learners independently, as above."""
     K = len(configs)
     if len(rngs) != K:
         raise ValueError("train_population needs one rng per config")
     full = [full_config(c) for c in configs]
     check_population_configs(full)
+    pbt_cfg = _pbt.check_pbt_config(pbt, K) if pbt is not None else None
     log_fns = list(log_fns) if log_fns is not None else [None] * K
     np_rngs = list(np_rngs) if np_rngs is not None else [None] * K
     learners = [Learner(configs[k], rngs[k], tables, eval_table, device, log_fns[k], eval_opp_params, np_rngs[k]) for k in range(K)]
     update_step = make_population_update_step([ln.config for ln in learners], learners[0].actor_forward_pass,
                                               [ln.optimizer for ln in learners])
+    controller = _pbt.PopulationBasedTraining(pbt_cfg, learners) if pbt_cfg is not None else None
     dev = learners[0].dev
     for i in range(full[0]["num_updates"]):
         batches = [ln.collect(i) for ln in learners]
@@ -320,6 +363,13 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
                            [b[2] for b in batches])
         torch.cuda.synchronize(dev)
         t_update = time.time() - t3
+        ranking = controller is not None and controller.due(i)
         for ln, (runner_state, loss_info) in zip(learners, outs):
-            ln.finish_iteration(i, runner_state, loss_info, t_update)
+            ln.finish_iteration(i, runner_state, loss_info, t_update, emit=not ranking)
+        if ranking:
+            controller.step(i, learners)
+            update_step = make_population_update_step([ln.config for ln in learners], learners[0].actor_forward_pass,
+                                                      [ln.optimizer for ln in learners])
+            for ln in learners:
+                ln.emit(ln.logs[-1])
     return [ln.finish() for ln in learners]
