@@ -1011,24 +1011,29 @@ int32_t brl_mlp_adam_step(brl_stream_t stream, void** b, const void* opaque, siz
     return check_launch("brl_mlp_adam_step");
 }
 
-int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+// brl_ppo_grad, and with `anchored` brl_ppo_grad_anchored: buffers [13] anchor logits, [14] kl_coef add the KL term
+static int32_t ppo_grad_impl(const char* what, bool anchored, brl_stream_t stream, void** b, const void* opaque, size_t len) {
     if (opaque == nullptr || len != sizeof(BrlPpoParams))
-        return fail(BRL_E_OPAQUE, "brl_ppo_grad: opaque must be one BrlPpoParams (%zu bytes), got %zu", sizeof(BrlPpoParams), len);
+        return fail(BRL_E_OPAQUE, "%s: opaque must be one BrlPpoParams (%zu bytes), got %zu", what, sizeof(BrlPpoParams), len);
     const BrlPpoParams* p = static_cast<const BrlPpoParams*>(opaque);
-    if (p->batch <= 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "brl_ppo_grad: batch must be in [1, 2^24]");
+    if (anchored && p->batch == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL
+    if (p->batch <= 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "%s: batch must be in [1, 2^24]", what);
     static const char* names[] = {"obs", "blob", "scratch", "index", "mask", "action", "old_log_prob", "old_value", "advantages",
-                                  "targets", "grads", "stats", "acc"};
-    const int32_t rc = check_buffers("brl_ppo_grad", b, names, 13, 1u << 3, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 10);
+                                  "targets", "grads", "stats", "acc", "anchor_logits", "kl_coef"};
+    const int32_t rc = check_buffers(what, b, names, anchored ? 15 : 13, 1u << 3, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 10);
     if (rc != BRL_OK) return rc;
-    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad: cuTensorMapEncodeTiled not available from the driver");
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "%s: cuTensorMapEncodeTiled not available from the driver", what);
     cudaStream_t s = (cudaStream_t)stream;
     // 3. loss head + its backward (src/update.py:97-162)
     struct PpoHead {
         void** b;
         BrlPpoParams params;
         bool defer_illegal;
+        PpoAnchor anchor;
     };
-    PpoHead head{b, *p, p->illegal_l2_coef == 0.0f};  // only the logged statistic needs the spectral norm: off the critical path
+    // only the logged statistic needs the spectral norm: off the critical path
+    PpoHead head{b, *p, p->illegal_l2_coef == 0.0f, PpoAnchor{}};
+    if (anchored) head.anchor = PpoAnchor{static_cast<const float*>(b[13]), nullptr, static_cast<const float*>(b[14])};
     head.params.flags &= (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
     head.params.reserved = 0;
     const bool skip_illegal = head.defer_illegal && !(p->flags & BRL_PPO_ILLEGAL_STAT);  // statistic not asked for: stats[6] = NaN
@@ -1036,7 +1041,8 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
         const PpoHead& h = *static_cast<const PpoHead*>(ctx);
         void* loss_buffers[13] = {const_cast<float*>(io.logits), const_cast<float*>(io.value), h.b[3], h.b[4], h.b[5], h.b[6], h.b[7],
                                   h.b[8], h.b[9], io.dlogits, io.dvalue, h.b[11], h.b[12]};
-        return launch_ppo_loss(st, loss_buffers, &h.params, io.dz_hi, io.dz_lo, /*acc_zeroed=*/true, h.defer_illegal);
+        return launch_ppo_loss(st, loss_buffers, &h.params, io.dz_hi, io.dz_lo, /*acc_zeroed=*/true, h.defer_illegal,
+                               h.anchor.coef ? &h.anchor : nullptr);
     };
     TrainMinibatch t{};
     t.obs = b[0];
@@ -1060,10 +1066,18 @@ int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t l
         t.gram = &gram;
         t.n_gram = gram_blocks(p->batch, 1024);
     }
-    t.what = "brl_ppo_grad";
+    t.what = what;
     t.loss_head = ppo_head;
     t.ctx = &head;
     return launch_train_minibatch(s, t);
+}
+
+int32_t brl_ppo_grad(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    return ppo_grad_impl("brl_ppo_grad", false, stream, b, opaque, len);
+}
+
+int32_t brl_ppo_grad_anchored(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    return ppo_grad_impl("brl_ppo_grad_anchored", true, stream, b, opaque, len);
 }
 
 // ---- K learners, one optimizer step each, in the launches of one -------------------------------------------------------
@@ -1076,19 +1090,21 @@ int64_t brl_ppo_grad_grouped_scratch_bytes(int64_t n_learners, int64_t batch) {
     return (int64_t)(grouped_ready_offset(n_learners, batch) + n_learners * ready_words(batch) * sizeof(uint32_t));
 }
 
-int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+// brl_ppo_grad_grouped, and with `anchored` brl_ppo_grad_grouped_anchored: buffers [7] anchor logits table, [8] kl_coef[K]
+static int32_t ppo_grad_grouped_impl(const char* what, bool anchored, brl_stream_t stream, void** b, const void* opaque, size_t len) {
     if (opaque == nullptr || len != sizeof(BrlPpoGroupedParams))
-        return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: opaque must be one BrlPpoGroupedParams (%zu bytes), got %zu",
-                    sizeof(BrlPpoGroupedParams), len);
+        return fail(BRL_E_OPAQUE, "%s: opaque must be one BrlPpoGroupedParams (%zu bytes), got %zu", what, sizeof(BrlPpoGroupedParams),
+                    len);
     const BrlPpoGroupedParams* p = static_cast<const BrlPpoGroupedParams*>(opaque);
     if (p->n_learners < 0 || p->n_learners > BRL_MAX_LEARNERS)
-        return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: n_learners must be in [0, %d]", BRL_MAX_LEARNERS);
-    if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "brl_ppo_grad_grouped: batch must be in [0, 2^24]");
+        return fail(BRL_E_OPAQUE, "%s: n_learners must be in [0, %d]", what, BRL_MAX_LEARNERS);
+    if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "%s: batch must be in [0, 2^24]", what);
     if (p->n_learners == 0 || p->batch == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL
-    static const char* names[] = {"traj", "coefs", "blob", "scratch", "grads", "stats", "acc"};
-    const int32_t rc = check_buffers("brl_ppo_grad_grouped", b, names, 7, 0, 1u << 0 | 1u << 2 | 1u << 3 | 1u << 4 | 1u << 6);
+    static const char* names[] = {"traj", "coefs", "blob", "scratch", "grads", "stats", "acc", "anchor_logits", "kl_coef"};
+    const int32_t rc = check_buffers(what, b, names, anchored ? 9 : 7, 0, 1u << 0 | 1u << 2 | 1u << 3 | 1u << 4 | 1u << 6);
     if (rc != BRL_OK) return rc;
-    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "brl_ppo_grad_grouped: cuTensorMapEncodeTiled not available from the driver");
+    if (encode_fn() == nullptr) return fail(BRL_E_LAUNCH, "%s: cuTensorMapEncodeTiled not available from the driver", what);
+    PpoAnchor anchor{nullptr, static_cast<const long long*>(anchored ? b[7] : nullptr), static_cast<const float*>(anchored ? b[8] : nullptr)};
     PpoGroupIO io{};  // the loss heads' arguments but the forward outputs, which launch_train_minibatch hands to the head
     io.traj = static_cast<const long long*>(b[0]);
     io.coefs = static_cast<const float*>(b[1]);
@@ -1098,6 +1114,7 @@ int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, 
     io.batch = p->batch;
     io.K = p->n_learners;
     io.flags = p->flags & (BRL_PPO_VALUE_CLIPPING | BRL_PPO_REWARD_SCALING | BRL_PPO_UNMASKED_POLICY | BRL_PPO_ILLEGAL_STAT);
+    io.anchor = anchored ? &anchor : nullptr;
     auto ppo_heads = [](cudaStream_t st, const TrainHeadIO& head, const void* ctx) -> int32_t {
         PpoGroupIO io = *static_cast<const PpoGroupIO*>(ctx);
         io.head = head;
@@ -1114,11 +1131,19 @@ int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, 
     t.zero = b[6];
     t.zero_bytes = 16 * sizeof(double);
     t.tune = p->reserved & ~8;  // the tile trace (tune bit 3) records one learner's launches
-    t.what = "brl_ppo_grad_grouped";
+    t.what = what;
     t.loss_head = ppo_heads;
     t.ctx = &io;
     t.group = &group;
     return launch_train_minibatch((cudaStream_t)stream, t);
+}
+
+int32_t brl_ppo_grad_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    return ppo_grad_grouped_impl("brl_ppo_grad_grouped", false, stream, b, opaque, len);
+}
+
+int32_t brl_ppo_grad_grouped_anchored(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    return ppo_grad_grouped_impl("brl_ppo_grad_grouped_anchored", true, stream, b, opaque, len);
 }
 
 int32_t brl_mlp_adam_step_grouped(brl_stream_t stream, void** b, const void* opaque, size_t len) {

@@ -41,7 +41,7 @@ struct PpoArgs {
 };
 
 // acc slots
-enum { kAccAdv = 0, kAccAdv2, kAccIll, kAccActor, kAccValue, kAccEnt, kAccKl, kAccClip, kAccGramTicket = 13, kAccTicket = 15 };
+enum { kAccAdv = 0, kAccAdv2, kAccIll, kAccActor, kAccValue, kAccEnt, kAccKl, kAccClip, kAccAnchorKl, kAccGramTicket = 13, kAccTicket = 15 };
 static_assert(128 + 40 * 8 <= 512 && 512 + kGramBlocks * kGramN * 4 <= BRL_PPO_SCRATCH_BYTES, "scratch layout");
 static_assert(kAccGramTicket == 13, "gram_args_at (ppo_gram.cuh) places the Gram ticket in f64 13");
 
@@ -188,9 +188,25 @@ __device__ __forceinline__ void ppo_finalize(const PpoArgs& a) {
     else if (!a.defer_illegal) a.stats[6] = ill;
     a.stats[7] = 0.0f;
 }
+// ... and with an anchor: stats[7] = mean_b KL_b, and its term in the total
+__device__ __forceinline__ void ppo_finalize_anchor(const PpoArgs& a, float kl_coef) {
+    const float kl = (float)(((const volatile double*)a.acc)[kAccAnchorKl] / (double)a.B);
+    a.stats[0] += kl_coef * kl;
+    a.stats[7] = kl;
+}
 
-template <class Args>  // PpoArgs, or PpoGroupArgs (blockIdx.y = learner)
-__global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass) {
+// The fixed reference policy of the KL term (k_ppo_loss<Args, PpoAnchor>): f32 anchor logits [total, 38] in the rows of the
+// flat trajectory, and the coefficient as a device scalar.  A group's learner k reads table[k] and coef[k].
+__device__ __forceinline__ PpoAnchor anchor_arg(const PpoAnchor& an) { return an; }
+template <class... Anchor>
+constexpr bool kAnchored = sizeof...(Anchor) != 0;  // (a namespace-scope constant: a local one perturbs the plain kernel's code)
+
+// Anchor = (nothing), or PpoAnchor: the anchored instantiation (brl_ppo_grad_anchored) adds coef * mean_b KL(pi(.|s_b) ||
+// alpha(.|s_b)), alpha = the anchor's softmax over the policy's own action set (the legal actions, or all 38 with
+// BRL_PPO_UNMASKED_POLICY): d / d logit_j = coef / B * pi_j (log pi_j - log alpha_j - KL_b) on the set, 0 elsewhere, with
+// 0 log 0 := 0.  The plain instantiation keeps the parameter list (Args, int) and compiles to the code it had before.
+template <class Args, class... Anchor>  // PpoArgs, or PpoGroupArgs (blockIdx.y = learner)
+__global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass, Anchor... an) {
     pdl_trigger();
     pdl_wait();
     const PpoArgs& a = learner_args(g);
@@ -213,6 +229,14 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
         v1[1] = lane < kA - 32 ? (float)a.spec[33 + lane] : 0.0f;
     }
     double s_actor = 0.0, s_value = 0.0, s_ent = 0.0, s_kl = 0.0, s_clip = 0.0;
+    double s_akl = 0.0;  // sum of KL_b to the anchor
+    const float* anchor = nullptr;
+    float kl_coef = 0.0f;
+    if constexpr (kAnchored<Anchor...>) {
+        const PpoAnchor x = anchor_arg(an...);
+        anchor = x.table ? reinterpret_cast<const float*>(x.table[blockIdx.y]) : x.logits;
+        kl_coef = x.coef[x.table ? blockIdx.y : 0];
+    }
     for (int64_t b = warp; b < a.B; b += nw) {
         const int64_t src = a.index ? a.index[b] : b;
         Row r;
@@ -244,6 +268,24 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
         // d (coef * sigma_1 / 2) / d logits_j = coef / 2 * (t / sigma_1) * (x_j v_j - q_j t)
         float qi[2] = {r.in[0] && !r.legal[0] ? q[0] : 0.0f, r.in[1] && !r.legal[1] ? q[1] : 0.0f};
         const float t_i = ill_grad ? warp_sum(qi[0] * v1[0] + qi[1] * v1[1]) : 0.0f;
+        // KL to the anchor over the policy's action set: the anchor's log-softmax over that set, then
+        // KL_b = sum_j pi_j (log pi_j - log alpha_j) and its gradient
+        float kl_b = 0.0f, dkl[2] = {0.0f, 0.0f};
+        if constexpr (kAnchored<Anchor...>) {
+            const bool* sel = a.masked_policy ? r.legal : r.in;
+            float al[2];
+#pragma unroll
+            for (int k = 0; k < 2; ++k) al[k] = sel[k] ? anchor[src * kA + lane + 32 * k] : -INFINITY;
+            const float amx = warp_max(fmaxf(al[0], al[1]));
+            const float alse = amx + logf(warp_sum((sel[0] ? expf(al[0] - amx) : 0.0f) + (sel[1] ? expf(al[1] - amx) : 0.0f)));
+            float lr[2];
+#pragma unroll
+            for (int k = 0; k < 2; ++k) lr[k] = sel[k] && pol_p[k] > 0.0f ? pol_logp[k] - (al[k] - alse) : 0.0f;
+            kl_b = warp_sum(pol_p[0] * lr[0] + pol_p[1] * lr[1]);
+            const float c_kl = kl_coef * invB;
+#pragma unroll
+            for (int k = 0; k < 2; ++k) dkl[k] = sel[k] && pol_p[k] > 0.0f ? c_kl * pol_p[k] * (lr[k] - kl_b) : 0.0f;
+        }
         // d total / d logits
 #pragma unroll
         for (int k = 0; k < 2; ++k) {
@@ -252,6 +294,7 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
             float d = c_ratio * ((j == act ? 1.0f : 0.0f) - pol_p[k]);
             if (r.legal[k] && p[k] > 0.0f) d += a.ent_coef * invB * p[k] * (logp[k] + ent);  // -ent_coef * dH/dl
             if (ill_grad) d += a.ill_coef * 0.5f * (t_i / sigma) * (qi[k] * v1[k] - q[k] * t_i);
+            if constexpr (kAnchored<Anchor...>) d += dkl[k];
             a.dlogits[b * kA + j] = d;
             if (a.dz_hi) split_store(a, b * 64 + j, d);
         }
@@ -279,21 +322,25 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
             s_ent += (double)ent;
             s_kl += (double)((ratio - 1.0f) - logratio);
             s_clip += fabsf(ratio - 1.0f) > a.clip_eps ? 1.0 : 0.0;
+            if constexpr (kAnchored<Anchor...>) s_akl += (double)kl_b;
         }
     }
     // block-level sums first (one set of same-address f64 atomics per block, not per warp), then the last block to
     // arrive (ticket in acc[kAccTicket]) forms the statistics: no separate finalize launch
-    __shared__ double part[4][5];
+    constexpr int kSums = kAnchored<Anchor...> ? 6 : 5;  // the f64 sums: actor, value, entropy, approx KL, clip fraction (, anchor KL)
+    __shared__ double part[4][kSums];
     __shared__ bool last_block;
     const int w = threadIdx.x >> 5;
     if (lane == 0) {
         part[w][0] = s_actor; part[w][1] = s_value; part[w][2] = s_ent; part[w][3] = s_kl; part[w][4] = s_clip;
+        if constexpr (kAnchored<Anchor...>) part[w][5] = s_akl;
     }
     __syncthreads();
-    if (threadIdx.x < 5) {
+    if (threadIdx.x < kSums) {
         const int k = threadIdx.x;
         const double s = part[0][k] + part[1][k] + part[2][k] + part[3][k];
-        const int slot = k == 0 ? kAccActor : k == 1 ? kAccValue : k == 2 ? kAccEnt : k == 3 ? kAccKl : kAccClip;
+        int slot = k == 0 ? kAccActor : k == 1 ? kAccValue : k == 2 ? kAccEnt : k == 3 ? kAccKl : kAccClip;
+        if constexpr (kAnchored<Anchor...>) slot = k == 5 ? kAccAnchorKl : slot;
         atomicAdd(&a.acc[slot], s);
     }
     __threadfence();
@@ -306,6 +353,7 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
     if (last_block && threadIdx.x == 0) {
         __threadfence();
         ppo_finalize(a);
+        if constexpr (kAnchored<Anchor...>) ppo_finalize_anchor(a, kl_coef);
     }
 }
 
@@ -434,10 +482,10 @@ brl::GramArgs brl::gram_args(void** b, const BrlPpoParams* p, float* stat) {
 
 // The loss head's launches, for one learner (Args = PpoArgs, a = g) or K (PpoGroupArgs, a = g.a, one grid row per learner):
 // `flags` decoded into `a`, then the advantage prepass (reward scaling), the Gram kernel (none when `gram` is NULL) and
-// the loss kernel.
+// the loss kernel (with the KL term when `anchor` is set).
 template <class Args, class GA>
 static int32_t launch_ppo_chain(cudaStream_t s, const Args& g, PpoArgs& a, int32_t flags, unsigned K, void (*gram)(GA), const GA& ga,
-                                const char* what) {
+                                const PpoAnchor* anchor, const char* what) {
     a.value_clipping = (flags & BRL_PPO_VALUE_CLIPPING) != 0;
     a.reward_scaling = (flags & BRL_PPO_REWARD_SCALING) != 0;
     a.masked_policy = (flags & BRL_PPO_UNMASKED_POLICY) == 0;
@@ -450,12 +498,13 @@ static int32_t launch_ppo_chain(cudaStream_t s, const Args& g, PpoArgs& a, int32
         if (prepass) gram<<<gram_grid, 1024, 0, s>>>(ga);  // a plain launch may not be followed by a PDL one that skips it
         else launch_pdl(gram, gram_grid, dim3(1024), 0, s, ga);
     }
-    launch_pdl(k_ppo_loss<Args>, dim3(grid, K), dim3(128), 0, s, g, prepass);
+    if (anchor) launch_pdl(k_ppo_loss<Args, PpoAnchor>, dim3(grid, K), dim3(128), 0, s, g, prepass, *anchor);
+    else launch_pdl(k_ppo_loss<Args>, dim3(grid, K), dim3(128), 0, s, g, prepass);
     return check_launch(what);
 }
 
 int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* p, void* dz_hi, void* dz_lo, bool acc_zeroed,
-                             bool defer_illegal) {
+                             bool defer_illegal, const PpoAnchor* anchor) {
     if (p->batch <= 0) return fail(BRL_E_OPAQUE, "brl_ppo_loss: batch must be > 0");
     static const char* names[] = {"logits", "value", "index", "mask", "action", "old_log_prob", "old_value", "advantages",
                                   "targets", "dlogits", "dvalue", "stats", "scratch"};
@@ -491,7 +540,7 @@ int32_t brl::launch_ppo_loss(cudaStream_t stream, void** b, const BrlPpoParams* 
     if (!acc_zeroed && cudaMemsetAsync(a.acc, 0, 16 * sizeof(double), s) != cudaSuccess) return check_launch("brl_ppo_loss");
     const GramArgs g = a.skip_illegal ? GramArgs{} : brl::gram_args(b, p, nullptr);
     void (*gram)(GramArgs) = a.skip_illegal ? nullptr : a.defer_illegal ? k_ppo_gram_partial : k_ppo_illegal_gram;
-    return launch_ppo_chain(s, a, a, p->flags, 1u, gram, g, "brl_ppo_loss");
+    return launch_ppo_chain(s, a, a, p->flags, 1u, gram, g, anchor, "brl_ppo_loss");
 }
 
 extern "C" {
@@ -578,5 +627,5 @@ int32_t brl::launch_ppo_loss_grouped(cudaStream_t s, const PpoGroupIO& io) {
     g.acc_stride = BRL_PPO_SCRATCH_BYTES;
     g.illegal_stat = (io.flags & BRL_PPO_ILLEGAL_STAT) != 0;
     // the Gram kernel runs for every learner: each decides from its own coefficient whether it has work
-    return launch_ppo_chain(s, g, a, io.flags, (unsigned)io.K, k_ppo_gram_grouped, g, "brl_ppo_grad_grouped");
+    return launch_ppo_chain(s, g, a, io.flags, (unsigned)io.K, k_ppo_gram_grouped, g, io.anchor, io.anchor ? "brl_ppo_grad_grouped_anchored" : "brl_ppo_grad_grouped");
 }

@@ -77,8 +77,14 @@ int32_t launch_categorical(cudaStream_t stream, const float* logits, const unsig
 // defer_illegal (honoured only when illegal_l2_coef == 0): only the partial Gram matrices are formed before the loss kernel;
 // the caller runs gram_tail() itself later (brl_ppo_grad: a spare block of k_bias_grad) with gram_args(buffers, p, &stats[6])
 // and gram_blocks(batch, 1024) partials
+// anchor (brl_ppo_grad_anchored): also the KL term to a fixed reference policy (stats[7] = its mean over the minibatch)
+struct PpoAnchor {
+    const float* logits;     // f32 [total, 38]: the anchor's logits in the rows of the flat trajectory (solo)
+    const long long* table;  // [K] device addresses of each learner's anchor logits (grouped; NULL = solo)
+    const float* coef;       // f32 kl_coef: [1] solo, [K] grouped (device scalars)
+};
 int32_t launch_ppo_loss(cudaStream_t stream, void** buffers, const BrlPpoParams* p, void* dz_hi, void* dz_lo, bool acc_zeroed,
-                        bool defer_illegal);
+                        bool defer_illegal, const PpoAnchor* anchor = nullptr);
 struct GramArgs;
 GramArgs gram_args(void** loss_buffers, const BrlPpoParams* p, float* stat);
 int gram_blocks(int64_t batch, int threads);
@@ -140,6 +146,7 @@ struct PpoGroupIO {
     int64_t batch;
     int K;
     int32_t flags;
+    const PpoAnchor* anchor;  // brl_ppo_grad_grouped_anchored (NULL: no KL term)
 };
 int32_t launch_ppo_loss_grouped(cudaStream_t stream, const PpoGroupIO& io);
 

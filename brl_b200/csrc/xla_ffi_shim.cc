@@ -78,6 +78,8 @@
     X(brl_evaluate_match, "iiisooxooooooooooooooooooo") \
     X(brl_ppo_grad_grouped, "iiisoos") \
     X(brl_mlp_adam_step_grouped, "xixxix") \
+    X(brl_ppo_grad_anchored, "iisiiiiiiioosii") \
+    X(brl_ppo_grad_grouped_anchored, "iiisoosii") \
     /* end */
 
 namespace {

@@ -157,6 +157,12 @@ class ForwardPass:
         ops.policy_act_rows(obs_bf16, self._packed(params), self._scratch, mask, action, rows, log_prob, logits, sample=sample, seed=seed,
                             env_offset=env_offset, single_bf16=self.precision == "tc-bf16")
 
+    def forward_into(self, params, obs_bf16: torch.Tensor, logits: torch.Tensor, value: torch.Tensor) -> None:
+        """`apply` on a bf16 observation, written into caller buffers (f32 logits [n, 38], value [n]): one brl_mlp_forward.
+        The roll-out records a KL anchor's logits with it."""
+        self._ensure_scratch(obs_bf16.shape[0], obs_bf16.device)
+        ops.mlp_forward(obs_bf16, self._packed(params), self._scratch, logits, value, single_bf16=self.precision == "tc-bf16")
+
     def pack_into(self, params, blob: torch.Tensor) -> torch.Tensor:
         """re-pack `params` into the caller's fixed-address blob (a PackedParams: a device-to-device copy of its blob)"""
         if isinstance(params, PackedParams):

@@ -401,12 +401,20 @@ def mlp_train_scratch(batch: int, device) -> torch.Tensor:
     return torch.empty(_lib.load().brl_mlp_train_scratch_bytes(batch), dtype=torch.uint8, device=device)
 
 
+def _anchor_args(op, anchor_logits, kl_coef):
+    if (anchor_logits is None) != (kl_coef is None):
+        raise _lib.BrlError(f"{op}: anchor_logits and kl_coef go together")
+
+
 def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, adv, targets, grads, stats, acc, *, clip_eps,
              ent_coef, vf_coef, illegal_l2_coef=0.0, value_clipping=True, reward_scaling=False, masked_policy=True,
-             illegal_stat: bool = True, tune: int = 0) -> None:
+             illegal_stat: bool = True, tune: int = 0, anchor_logits: Optional[torch.Tensor] = None,
+             kl_coef: Optional[torch.Tensor] = None) -> None:
     """One minibatch of jax.value_and_grad(_loss_fn) (src/update.py:91-167): take(index), forward, loss, backward
     through the MLP on tcgen05 -> flat fp32 gradients (+ the loss statistics of `ppo_loss`).  `illegal_stat=False` (only
-    honoured with illegal_l2_coef == 0): skip the logged illegal_action_loss (stats[6] = NaN), ~19 us per call."""
+    honoured with illegal_l2_coef == 0): skip the logged illegal_action_loss (stats[6] = NaN), ~19 us per call.
+    `anchor_logits` (f32 [total, 38], an anchor net's logits for every trajectory row) with `kl_coef` (CUDA f32[1]): add
+    kl_coef * mean KL(policy || anchor) to the loss (brl_ppo_grad_anchored); stats[7] = that mean KL."""
     L = _lib.load()
     B = int(index.shape[0]) if index is not None else int(obs.shape[0])
     if obs.dtype == torch.bool:
@@ -417,10 +425,19 @@ def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, a
         raise _lib.BrlError("ppo_grad: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
     if grads.dtype != torch.float32 or grads.numel() != L.brl_mlp_num_params():
         raise _lib.BrlError("ppo_grad: grads must be the flat fp32 gradient buffer")
+    _anchor_args("ppo_grad", anchor_logits, kl_coef)
     p = _lib.BrlPpoParams(B, int(action.numel()), float(clip_eps), float(ent_coef), float(vf_coef), float(illegal_l2_coef),
                           flags, int(tune))
-    _call("brl_ppo_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(index), _ptr(mask), _ptr(action), _ptr(old_log_prob),
-                           _ptr(old_value), _ptr(adv), _ptr(targets), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+    buffers = [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(index), _ptr(mask), _ptr(action), _ptr(old_log_prob),
+               _ptr(old_value), _ptr(adv), _ptr(targets), _ptr(grads), _ptr(stats), _ptr(acc)]
+    if anchor_logits is None:
+        _call("brl_ppo_grad", buffers, p)
+        return
+    if anchor_logits.dtype != torch.float32 or anchor_logits.numel() != action.numel() * NUM_ACTIONS:
+        raise _lib.BrlError("ppo_grad: anchor_logits must be float32[total, 38] (one row per trajectory row)")
+    if kl_coef.dtype != torch.float32 or kl_coef.numel() != 1:
+        raise _lib.BrlError("ppo_grad: kl_coef must be a float32[1] device scalar")
+    _call("brl_ppo_grad_anchored", buffers + [_ptr(anchor_logits), _ptr(kl_coef)], p)
 
 
 # ---- population training: K learners' optimizer steps in the launches of one (brl_ppo_grad_grouped) ----------------------
@@ -443,12 +460,15 @@ def ppo_trajectory_row(obs, index, mask, action, old_log_prob, old_value, adv, t
 
 
 def ppo_grad_grouped(traj, coefs, blob, scratch, grads, stats, acc, *, batch: int, obs_dtype, value_clipping=True,
-                     reward_scaling=False, masked_policy=True, illegal_stat: bool = True, tune: int = 0) -> None:
+                     reward_scaling=False, masked_policy=True, illegal_stat: bool = True, tune: int = 0,
+                     anchor_logits: Optional[torch.Tensor] = None, kl_coef: Optional[torch.Tensor] = None) -> None:
     """`ppo_grad` for K learners in one set of launches.  traj: CUDA int64[K, 8] rows of `ppo_trajectory_row`; coefs: CUDA
     float32[K, 4] = (clip_eps, ent_coef, vf_coef, illegal_l2_coef) per learner; blob: uint8[K, mlp_train_blob_bytes];
     grads: float32[K, mlp_param_stride]; stats: float32[K, 8]; acc: float64[K, PPO_SCRATCH_BYTES / 8], whose row k holds
     learner k's |grads|^2 at element 14 on return.  Every learner's minibatch has `batch` rows and observations of
-    `obs_dtype`; learner k's results are bit-identical to `ppo_grad` with its own buffers and coefficients."""
+    `obs_dtype`; learner k's results are bit-identical to `ppo_grad` with its own buffers and coefficients.
+    `anchor_logits` (CUDA int64[K]: the device address of learner k's f32 anchor logits [total_k, 38]) with `kl_coef` (CUDA
+    float32[K]): each learner's KL term, as `ppo_grad(..., anchor_logits=, kl_coef=)` (brl_ppo_grad_grouped_anchored)."""
     L = _lib.load()
     K = int(traj.shape[0]) if traj.dim() == 2 else -1
     if traj.dtype != torch.int64 or traj.dim() != 2 or traj.shape[1] != 8:
@@ -466,8 +486,15 @@ def ppo_grad_grouped(traj, coefs, blob, scratch, grads, stats, acc, *, batch: in
                             "scratch ppo_grad_grouped_scratch_bytes(K, batch)")
     flags = _ppo_flags("ppo_grad_grouped", value_clipping=value_clipping, reward_scaling=reward_scaling, masked_policy=masked_policy,
                        illegal_stat=illegal_stat, obs_dtype=obs_dtype)
+    _anchor_args("ppo_grad_grouped", anchor_logits, kl_coef)
     p = _lib.BrlPpoGroupedParams(int(batch), K, flags, int(tune), 0)
-    _call("brl_ppo_grad_grouped", [_ptr(traj), _ptr(coefs), _ptr(blob), _ptr(scratch), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+    buffers = [_ptr(traj), _ptr(coefs), _ptr(blob), _ptr(scratch), _ptr(grads), _ptr(stats), _ptr(acc)]
+    if anchor_logits is None:
+        _call("brl_ppo_grad_grouped", buffers, p)
+        return
+    if anchor_logits.dtype != torch.int64 or anchor_logits.numel() != K or kl_coef.dtype != torch.float32 or kl_coef.numel() != K:
+        raise _lib.BrlError("ppo_grad_grouped: anchor_logits must be int64[K] device addresses, kl_coef float32[K]")
+    _call("brl_ppo_grad_grouped_anchored", buffers + [_ptr(anchor_logits), _ptr(kl_coef)], p)
 
 
 def mlp_adam_step_grouped(params, grads, m, v, acc, blob, *, steps, lrs, max_grad_norms, beta1=0.9, beta2=0.999,

@@ -20,11 +20,12 @@ from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
-# The hyperparameters an explore step may multiply: the loss coefficients and the optimizer's (read by the update step
-# and the optimizer, rebuilt after each change) and GAE's (read by calc_gae at every call).  Keys of
-# update.POPULATION_SHARED_KEYS fix shapes or launch flags and cannot differ between learners.
+# The hyperparameters an explore step may multiply: the loss coefficients (the KL anchor's among them) and the optimizer's
+# (read by the update step and the optimizer, rebuilt after each change) and GAE's (read by calc_gae at every call).  Keys
+# of update.POPULATION_SHARED_KEYS fix shapes or launch flags and cannot differ between learners.  A loser keeps its own
+# anchor net and takes the winner's anchor_kl_coef times the factor.
 PERTURBABLE_KEYS = ("lr", "ent_coef", "vf_coef", "clip_eps", "max_grad_norm", "illegal_action_l2norm_coef", "gamma",
-                    "gae_lambda")
+                    "gae_lambda", "anchor_kl_coef")
 
 METRICS = ("league", "score")
 

@@ -2,6 +2,11 @@
 update per iteration, with the per-iteration strength probes, the FSP / PFSP opponent
 league (ppo.py:392-470) and the DDS-table rotation (ppo.py:525-549).
 
+KL anchor (not in the reference): `anchor_model_path` names a fixed net of the actor's architecture (e.g. the SL model a
+run starts from) and `anchor_kl_coef` the weight of coef * mean KL(policy || anchor) in every minibatch's loss.  The
+roll-out records the anchor's logits, the update adds the term (a loss term: rewards, GAE and value targets are
+unchanged), and the log gains `train/anchor_kl`.  Unset (the default), every code path is the one without the feature.
+
 Everything heavy runs in the kernels behind `brl_b200.ops`; this file is the control
 plane only (config defaults, opponent selection, table rotation, logging hooks).  wandb,
 OmegaConf and the dataset download are out of scope (SURVEY 2): `log_fn` receives the same
@@ -11,6 +16,7 @@ DDS dataset cannot be downloaded offline).
 """
 from __future__ import annotations
 
+import math
 import os
 import pickle
 import time
@@ -48,7 +54,16 @@ def default_config() -> dict:
         num_prioritized_envs=100, gamma=1.0, gae_lambda=0.95, clip_eps=0.2, ent_coef=0.001, vf_coef=0.5,
         value_clipping=True, global_gradient_clipping=True, anneal_lr=False, reward_scaling=False, max_grad_norm=0.5,
         reward_scale=7600.0, actor_illegal_action_mask=True, actor_illegal_action_penalty=False,
-        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0)
+        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0, anchor_model_path=None, anchor_kl_coef=0.0)
+
+
+def check_anchor_config(config: dict) -> None:
+    """ValueError for an anchor_kl_coef that is negative or not a finite number, or non-zero without anchor_model_path"""
+    coef = config.get("anchor_kl_coef", 0.0)
+    if isinstance(coef, bool) or not isinstance(coef, (int, float, np.integer, np.floating)) or not math.isfinite(coef) or coef < 0:
+        raise ValueError(f"anchor_kl_coef must be a finite number >= 0; got {coef!r}")
+    if coef != 0 and not config.get("anchor_model_path"):
+        raise ValueError(f"anchor_kl_coef = {coef!r} needs an anchor net: set anchor_model_path")
 
 
 def params_to_host(params) -> dict:
@@ -100,6 +115,7 @@ class Learner:
                  np_rng: Optional[np.random.Generator] = None, forward_pass_factory=None):
         make_fp = forward_pass_factory or make_forward_pass
         self.config = config = full_config(config)
+        check_anchor_config(config)
         self.log_fn = log_fn
         self.np_rng = np_rng or np.random.default_rng(config["seed"])
         self.dev = dev = torch.device(device)
@@ -135,8 +151,15 @@ class Learner:
                                                                                                         eval_opp_params)
 
         opp_forward_pass = make_fp(config["opp_activation"], config["opp_model_type"])
+        # the KL anchor: a fixed net of the actor's architecture, this learner's own (PBT's adopt keeps it)
+        self.anchor_params, anchor_forward_pass = None, None
+        if config["anchor_model_path"]:
+            self.anchor_params = load_params(config["anchor_model_path"], dev)
+            anchor_forward_pass = make_fp(config["actor_activation"], config["actor_model_type"])
+        self.anchor_logits = None  # the latest roll-out's anchor logits [num_steps, num_envs, 38]
         self.envs = [BridgeBidding(table=t, device=dev) for t in tables]                              # ppo.py:296-303
-        self.roll_outs = [make_roll_out(config, env, self.actor_forward_pass, opp_forward_pass) for env in self.envs]
+        self.roll_outs = [make_roll_out(config, env, self.actor_forward_pass, opp_forward_pass, anchor_forward_pass)
+                          for env in self.envs]
         self.calc_gae = make_calc_gae(config, self.actor_forward_pass)
 
         rng, _rng = brandom.split(rng)
@@ -223,7 +246,8 @@ class Learner:
         (self.imp_opp_before, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng)
         torch.cuda.synchronize(dev)
         t1 = time.time()
-        runner_state, traj_batch = self.roll_out(runner_state, self.opp_params)                   # ppo.py:472-475
+        runner_state, traj_batch = self.roll_out(runner_state, self.opp_params, anchor_params=self.anchor_params)  # :472-475
+        self.anchor_logits = self.roll_out.anchor_logits
         torch.cuda.synchronize(dev)
         t2 = time.time()
         advantages, targets = self.calc_gae(runner_state, traj_batch)                             # ppo.py:477
@@ -233,9 +257,14 @@ class Learner:
         self.runner_state = runner_state
         return traj_batch, advantages, targets
 
-    def finish_iteration(self, i: int, runner_state, loss_info, t_update: float, emit: bool = True) -> dict:
+    def update_kwargs(self) -> dict:
+        """the update step's keywords for the latest roll-out: its anchor logits when this learner has an anchor"""
+        return {} if self.anchor_params is None else {"anchor_logits": self.anchor_logits}
+
+    def finish_iteration(self, i: int, runner_state, loss_info, t_update: float, emit: bool = True, anchor_kl=None) -> dict:
         """Iteration i after the update (ppo.py:479-549): the strength probe, the log, the table rotation.  `emit=False`
-        leaves the log_fn call to the caller (`emit`), which adds entries to the log first."""
+        leaves the log_fn call to the caller (`emit`), which adds entries to the log first.  `anchor_kl`: the update's
+        per-minibatch KL to the anchor, [update_epochs, num_minibatches], logged as train/anchor_kl when there is an anchor."""
         config, dev = self.config, self.dev
         self.runner_state = runner_state
         (imp_opp_after, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, self.eval_rng)
@@ -252,6 +281,8 @@ class Learner:
             "board_num": board_num, "steps": self.steps,
             "time/eval": self.t_eval, "time/rollout": self.t_rollout, "time/calc_gae": self.t_gae, "time/update": t_update,
         }
+        if self.anchor_params is not None:
+            log["train/anchor_kl"] = float(anchor_kl[-1][-1])
         log.update(self.eval_log)
         self.logs.append(log)
         if emit:
@@ -278,7 +309,8 @@ class Learner:
         """PBT's exploit and explore: take `src`'s parameters and Adam state (device copies into this learner's own
         buffers, on the current stream) and set the config `values`, rebuilding the optimizer that captured them.  The
         update step holds the loss coefficients and optimizers and is the caller's to rebuild.  Env state, rollout key,
-        table rotation, zoo and save directory stay this learner's; a self-play opponent becomes the new parameters."""
+        table rotation, zoo, KL anchor and save directory stay this learner's; a self-play opponent becomes the new
+        parameters."""
         params, opt_state = self.runner_state[:2]
         src_params, src_state = src.runner_state[:2]
         for name in LAYERS:
@@ -316,9 +348,10 @@ def train(config: dict, rng: int, tables: Optional[Sequence] = None, eval_table=
     for i in range(learner.config["num_updates"]):
         traj_batch, advantages, targets = learner.collect(i)
         t3 = time.time()
-        runner_state, loss_info = update_step(learner.runner_state, traj_batch, advantages, targets)  # ppo.py:479-484
+        runner_state, loss_info = update_step(learner.runner_state, traj_batch, advantages, targets,
+                                              **learner.update_kwargs())                          # ppo.py:479-484
         torch.cuda.synchronize(learner.dev)
-        learner.finish_iteration(i, runner_state, loss_info, time.time() - t3)
+        learner.finish_iteration(i, runner_state, loss_info, time.time() - t3, anchor_kl=getattr(update_step, "anchor_kl", None))
     return learner.finish()
 
 
@@ -342,12 +375,21 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
     pbt/rank (0 = fittest), pbt/parent (the learner copied, or -1) and pbt/<key> for each perturbed key before log_fns
     see them, and with save_model each learner's save directory gets a pbt_lineage.json.  ValueError (before any device work) for K < 2, a quantile outside (0, 0.5], a perturbed key that
     default_config() does not know or that the population shares, and the other bad options pbt.check_pbt_config lists.
-    None (the default) trains the learners independently, as above."""
+    None (the default) trains the learners independently, as above.
+
+    KL anchors: each learner has its own anchor net (anchor_model_path) and coefficient (anchor_kl_coef, which PBT may
+    perturb); either every learner has an anchor or none has (ValueError naming anchor_model_path)."""
     K = len(configs)
     if len(rngs) != K:
         raise ValueError("train_population needs one rng per config")
     full = [full_config(c) for c in configs]
     check_population_configs(full)
+    for c in full:
+        check_anchor_config(c)
+    anchored = [bool(c["anchor_model_path"]) for c in full]
+    if any(anchored) and not all(anchored):
+        raise ValueError(f"population learners must all have a KL anchor or none: anchor_model_path is set for learners "
+                         f"{[k for k in range(K) if anchored[k]]} only")
     pbt_cfg = _pbt.check_pbt_config(pbt, K) if pbt is not None else None
     log_fns = list(log_fns) if log_fns is not None else [None] * K
     np_rngs = list(np_rngs) if np_rngs is not None else [None] * K
@@ -359,13 +401,15 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
     for i in range(full[0]["num_updates"]):
         batches = [ln.collect(i) for ln in learners]
         t3 = time.time()
+        anchor = {"anchor_logits": [ln.anchor_logits for ln in learners]} if any(anchored) else {}
         outs = update_step([ln.runner_state for ln in learners], [b[0] for b in batches], [b[1] for b in batches],
-                           [b[2] for b in batches])
+                           [b[2] for b in batches], **anchor)
         torch.cuda.synchronize(dev)
         t_update = time.time() - t3
         ranking = controller is not None and controller.due(i)
-        for ln, (runner_state, loss_info) in zip(learners, outs):
-            ln.finish_iteration(i, runner_state, loss_info, t_update, emit=not ranking)
+        anchor_kl = getattr(update_step, "anchor_kl", None) or [None] * K
+        for k, (ln, (runner_state, loss_info)) in enumerate(zip(learners, outs)):
+            ln.finish_iteration(i, runner_state, loss_info, t_update, emit=not ranking, anchor_kl=anchor_kl[k])
         if ranking:
             controller.step(i, learners)
             update_step = make_population_update_step([ln.config for ln in learners], learners[0].actor_forward_pass,

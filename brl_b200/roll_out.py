@@ -14,6 +14,12 @@ replay (an opponent given as models.PackedParams, e.g. from zoo.ModelZoo, is cop
 per-rollout PRNG key is a device word XORed into every captured sampling seed (BRL_F_SEED_SALT).  The returned
 trajectory then aliases the graph's buffers: it is valid until the next call of the same roll_out.
 `BRL_ROLLOUT_GRAPH=0` (or `trace=`) selects the plain launch path.
+
+Anchor (a KL-anchored PPO run, ppo.py `anchor_model_path`): `roll_out(runner_state, opp_params, anchor_params)` also runs
+the anchor net on every step's observation (one `brl_mlp_forward` on the same bf16 `obs[t]`) into f32
+`roll_out.anchor_logits[T, n, 38]`, which the update's KL term reads.  The buffer belongs to the roll-out and, like the
+trajectory, stays valid until the next call.  Anchored and plain calls keep separate buffers and CUDA graphs; the anchor
+is packed into its own fixed-address blob before an anchored replay.
 """
 from __future__ import annotations
 
@@ -25,7 +31,7 @@ import torch
 from . import ops
 from . import random as brandom
 from .env import State
-from .utils import auto_reset, single_play_step_free_run, single_play_step_two_policy_commpetitive
+from .utils import WithOutputs, auto_reset, single_play_step_free_run, single_play_step_two_policy_commpetitive
 
 _GRAPH_MIN_ENVS = 4096  # BRL_F_SEED_SALT lives in the fused forward launch
 _CAPTURE_KEY = 0x5EED    # host key the captured seeds are split from; the per-rollout key is the device salt
@@ -83,7 +89,7 @@ class _Buffers:
             self.player[0].copy_(env_state.current_player)
 
 
-def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
+def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forward_pass=None):
     masked = bool(config["actor_illegal_action_mask"])
     if not masked and not config.get("actor_illegal_action_penalty", False):
         raise ValueError("one of actor_illegal_action_mask / actor_illegal_action_penalty must be set (src/roll_out.py:24-39)")
@@ -96,9 +102,10 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
     T = int(config["num_steps"])
     scale = float(config["reward_scale"])
     obs_dtype = getattr(actor_forward_pass, "input_dtype", torch.float32)
-    cache = {}  # n -> dict(buf, graph, blobs, salt, ...)
+    cache = {}  # (n, anchored) -> dict(buf, graph, blobs, salt, anchor_logits, ...)
+    out = {"anchor_logits": None}
 
-    def body(buf, params, opp_params, rng, trace):
+    def body(buf, params, opp_params, rng, trace, anchor=None):
         """the T steps of src/roll_out.py:49-108 on `buf`"""
         step_fn = make_step_fn(step_fn=auto_reset(env.step, env.init), actor_forward_pass=actor_forward_pass,
                                actor_params=params, opp_forward_pass=opp_forward_pass, opp_params=opp_params)
@@ -108,6 +115,9 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
             rng, _rng = brandom.split(rng)
             actor_forward_pass.act(params, buf.obs[t], buf.mask[t] if masked else None, buf.action[t], buf.log_prob[t],
                                    buf.value[t], sample=True, seed=_rng, env_offset=getattr(env, "env_offset", 0))  # :73-81
+            if anchor is not None:  # the anchor's logits on the observation the actor just saw
+                anchor_params, anchor_logits, anchor_value = anchor
+                anchor_forward_pass.forward_into(anchor_params, buf.obs[t], anchor_logits[t], anchor_value)
             rng, _rng = brandom.split(rng)
             cur = step_fn(cur, buf.action[t], _rng, out_state=buf.state(env, t + 1))                                # :84
             # reward = rewards[actor] / scale with actor = the player who was to act BEFORE the quad step (still in the
@@ -121,18 +131,27 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
                           log_prob=buf.log_prob, obs=buf.obs[:T], legal_action_mask=buf.mask[:T].view(torch.bool))
         return (params, opt_state, cur, cur.observation, total, rng), traj
 
-    def roll_out(runner_state, opp_params, trace=None, graph_seeding=False):
-        """`trace` (tests): a list that receives every sub-step action tensor; forces the plain launch path.
-        `graph_seeding` (tests): plain launches with exactly the seeds a graph replay uses (captured constants XOR the
-        per-rollout salt), so that a graph replay can be compared bit for bit with a traced, oracle-checked run."""
+    def roll_out(runner_state, opp_params, anchor_params=None, trace=None, graph_seeding=False):
+        """`anchor_params`: also record the anchor net's logits of every step in `roll_out.anchor_logits` (needs
+        `anchor_forward_pass`).  `trace` (tests): a list that receives every sub-step action tensor; forces the plain
+        launch path.  `graph_seeding` (tests): plain launches with exactly the seeds a graph replay uses (captured constants
+        XOR the per-rollout salt), so that a graph replay can be compared bit for bit with a traced, oracle-checked run."""
         params, opt_state, env_state, last_obs, terminated_count, rng = runner_state
         n, dev = env_state.num_envs, env.device
+        anchored = anchor_params is not None
+        if anchored and anchor_forward_pass is None:
+            raise ValueError("roll_out got anchor_params, but make_roll_out was given no anchor_forward_pass")
         use_graph = trace is None and not graph_seeding and n >= _GRAPH_MIN_ENVS and \
             os.environ.get("BRL_ROLLOUT_GRAPH", "1") != "0" and \
-            hasattr(actor_forward_pass, "pack_into") and hasattr(opp_forward_pass, "pack_into")  # tensor-core nets only
-        c = cache.get(n)
+            hasattr(actor_forward_pass, "pack_into") and hasattr(opp_forward_pass, "pack_into") and \
+            (not anchored or hasattr(anchor_forward_pass, "pack_into"))  # tensor-core nets only
+        c = cache.get((n, anchored))
         if c is None:
-            c = cache[n] = {"buf": _Buffers(T, n, dev, obs_dtype), "graph": None}
+            c = cache[(n, anchored)] = {"buf": _Buffers(T, n, dev, obs_dtype), "graph": None}
+            if anchored:
+                c["anchor_logits"] = torch.empty((T, n, ops.NUM_ACTIONS), dtype=torch.float32, device=dev)
+                c["anchor_value"] = torch.empty(n, dtype=torch.float32, device=dev)
+        out["anchor_logits"] = c["anchor_logits"] if anchored else None
         buf = c["buf"]
         buf.load(env_state, last_obs)
         buf.count.zero_()
@@ -144,8 +163,9 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
                 salt = torch.tensor([key - (1 << 64) if key >= (1 << 63) else key], dtype=torch.int64, device=dev)
                 body_rng = _CAPTURE_KEY
             actor_forward_pass.seed_salt = opp_forward_pass.seed_salt = salt
+            anchor = (anchor_params, c["anchor_logits"], c["anchor_value"]) if anchored else None
             try:
-                cur, body_rng = body(buf, params, opp_params, body_rng, trace)
+                cur, body_rng = body(buf, params, opp_params, body_rng, trace, anchor)
             finally:
                 actor_forward_pass.seed_salt, opp_forward_pass.seed_salt = prev
             return finish(buf, params, opt_state, cur, terminated_count, rng if graph_seeding else body_rng)
@@ -161,6 +181,12 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
         fixed_a, fixed_o = {"_brl_packed_fixed": c["blobs"][0]}, {"_brl_packed_fixed": c["blobs"][1]}
         actor_forward_pass.pack_into(params, c["blobs"][0])
         (opp_forward_pass if opp_params is not params else actor_forward_pass).pack_into(opp_params, c["blobs"][1])
+        anchor = None
+        if anchored:
+            if "anchor_blob" not in c:
+                c["anchor_blob"] = torch.empty(ops._lib.load().brl_mlp_packed_bytes(), dtype=torch.uint8, device=dev)
+            anchor_forward_pass.pack_into(anchor_params, c["anchor_blob"])
+            anchor = ({"_brl_packed_fixed": c["anchor_blob"]}, c["anchor_logits"], c["anchor_value"])
         if c["graph"] is None:
             prev = (getattr(actor_forward_pass, "seed_salt", None), getattr(opp_forward_pass, "seed_salt", None))
             actor_forward_pass.seed_salt = opp_forward_pass.seed_salt = c["salt"]  # baked into the captured launches only
@@ -169,13 +195,13 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
             side.wait_stream(torch.cuda.current_stream(dev))
             try:
                 with torch.cuda.stream(side):
-                    body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None)  # warm-up: lazy allocations (scratch), attribute calls
+                    body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor)  # warm-up: lazy allocations (scratch), attribute calls
                     buf.packed.copy_(saved[0]); buf.obs[0].copy_(saved[1]); buf.mask[0].copy_(saved[2]); buf.player[0].copy_(saved[3])
                     buf.count.zero_()
                     side.synchronize()
                     g = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g, stream=side):
-                        body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None)
+                        body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor)
             finally:
                 actor_forward_pass.seed_salt, opp_forward_pass.seed_salt = prev
             torch.cuda.current_stream(dev).wait_stream(side)
@@ -186,4 +212,4 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass):
         cur = buf.state(env, T)
         return finish(buf, params, opt_state, cur, terminated_count, rng)
 
-    return roll_out
+    return WithOutputs(roll_out, out)

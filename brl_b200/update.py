@@ -7,7 +7,11 @@ backward GEMMs all in hand-written kernels on tcgen05 (csrc/brl_mlp_train.cu, th
 gradients) -- then `brl_mlp_adam_step` (clip + Adam + refresh of the kernels' weight layout in one pass).  No library
 GEMM, no autograd tape.  (The cuBLAS-fp32 + autograd cross-check of this path is scripts/torch_baseline.py.)
 Functional semantics are kept: the caller's `params` / `opt_state` are not modified (ppo.py
-keeps the pre-update params as `opp_params`), a new flat copy is updated and returned."""
+keeps the pre-update params as `opp_params`), a new flat copy is updated and returned.
+
+KL anchor: `update_step(..., anchor_logits=)` with the roll-out's anchor logits [T, n, 38] adds config["anchor_kl_coef"] *
+mean KL(policy || anchor) to every minibatch's loss (brl_ppo_grad_anchored); the per-minibatch KL, [update_epochs,
+num_minibatches], is then `update_step.anchor_kl` after the call (None without an anchor)."""
 from __future__ import annotations
 
 import torch
@@ -15,6 +19,7 @@ import torch
 from . import _lib, ops
 from . import random as brandom
 from .optim import OptState, flatten_params, update_mlp_grouped_
+from .utils import WithOutputs
 
 _STAT_NAMES = ("total_loss", "value_loss", "loss_actor", "entropy", "approx_kl", "clipflacs", "illegal_action_loss")
 
@@ -55,6 +60,13 @@ def _flat_rollout(traj_batch, advantages, targets, batch_size):
             targets.reshape(batch_size).contiguous())
 
 
+def _flat_anchor(anchor_logits, batch_size):
+    """the roll-out's anchor logits [T, n, 38] as the f32 [T * n, 38] rows of the flat rollout"""
+    if anchor_logits.dtype != torch.float32 or anchor_logits.numel() != batch_size * ops.NUM_ACTIONS:
+        raise ValueError("anchor_logits must be the roll-out's float32 [num_steps, num_envs, 38] anchor logits")
+    return anchor_logits.reshape(batch_size, ops.NUM_ACTIONS).contiguous()
+
+
 def _permutation(permutation_fn, rng, batch_size, device):
     """One epoch's minibatch order (src/update.py:193): `permutation_fn`, or torch.randperm seeded by the key."""
     if permutation_fn is not None:
@@ -77,12 +89,18 @@ def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None)
     (src/update.py:193); default: torch.randperm seeded by the key (tests inject a fixed one)."""
     flags, coefs, stat_mode, tune = _loss_settings(config, actor_forward_pass, "make_update_step")
     cfg = dict(zip(("clip_eps", "ent_coef", "vf_coef", "illegal_l2_coef"), coefs), **flags)
+    kl_coef = float(config.get("anchor_kl_coef", 0.0))
+    out = {"anchor_kl": None}
 
-    def update_step(runner_state, traj_batch, advantages, targets):
+    def update_step(runner_state, traj_batch, advantages, targets, anchor_logits=None):
         params, opt_state, env_state, last_obs, terminated_count, rng = runner_state
         dev = advantages.device
         nmb, mbs = int(config["num_minibatches"]), int(config["minibatch_size"])
         obs, mask, action, old_lp, old_v, adv, tgt = _flat_rollout(traj_batch, advantages, targets, nmb * mbs)
+        anchor = {}
+        if anchor_logits is not None:
+            anchor = dict(anchor_logits=_flat_anchor(anchor_logits, nmb * mbs),
+                          kl_coef=torch.tensor([kl_coef], dtype=torch.float32).to(dev))
 
         flat_p, new_params = flatten_params(params)
         if opt_state is None:
@@ -100,11 +118,12 @@ def make_update_step(config, actor_forward_pass, optimizer, permutation_fn=None)
             for mb in range(nmb):                                                  # src/update.py:207-209
                 ops.ppo_grad(obs, blob, scratch, perm[mb * mbs:(mb + 1) * mbs], mask, action, old_lp, old_v, adv, tgt,
                              flat_g, stats_all[epoch, mb], acc, tune=tune, illegal_stat=stat_mode == "all" or mb == nmb - 1,
-                             **cfg)                                                # src/update.py:164-167
+                             **cfg, **anchor)                                      # src/update.py:164-167
                 state = optimizer.update_mlp_(flat_p, flat_g, state, acc[14:15], blob)  # src/update.py:168-169
+        out["anchor_kl"] = stats_all[:, :, 7] if anchor else None
         return (new_params, state, env_state, last_obs, terminated_count, rng), _loss_info(stats_all)
 
-    return update_step
+    return WithOutputs(update_step, out)
 
 
 # Keys every learner of a population must share: they fix the shapes of the stacked buffers and the flags and tile widths
@@ -132,7 +151,9 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
     learner and returns K `(runner_state, loss_info)` pairs, each what `make_update_step(configs[k], ...)` returns for
     that learner: every learner draws its permutations from its own key, and its parameters, optimizer state and loss
     statistics are bit-identical to its solo update.  The stacked parameter, gradient, moment and blob buffers of the
-    whole update are owned here; the returned params / opt_state are views into them."""
+    whole update are owned here; the returned params / opt_state are views into them.  `anchor_logits=`: one roll-out's
+    anchor logits per learner (every learner has an anchor or none has); `update_step.anchor_kl` is then a list of each
+    learner's [update_epochs, num_minibatches] KL."""
     configs = list(configs)
     check_population_configs(configs)
     if len(optimizers) != len(configs):
@@ -142,12 +163,22 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
     settings = [_loss_settings(c, actor_forward_pass, "make_population_update_step") for c in configs]
     flags, _, stat_mode, tune = settings[0]  # shared keys: equal for every learner
     coef_rows = [coefs for _, coefs, _, _ in settings]
+    kl_coefs = [float(c.get("anchor_kl_coef", 0.0)) for c in configs]
     c0 = configs[0]
     K = len(configs)
+    out = {"anchor_kl": None}
 
-    def update_step(runner_states, traj_batches, advantages, targets):
+    def update_step(runner_states, traj_batches, advantages, targets, anchor_logits=None):
         if not (len(runner_states) == len(traj_batches) == len(advantages) == len(targets) == K):
             raise ValueError(f"update_step needs {K} runner states, trajectories, advantages and targets")
+        if anchor_logits is not None:
+            if len(anchor_logits) != K:
+                raise ValueError(f"update_step needs {K} anchor logits")
+            if any(a is None for a in anchor_logits):
+                if all(a is None for a in anchor_logits):
+                    anchor_logits = None
+                else:
+                    raise ValueError("population learners must all have a KL anchor (anchor_model_path) or none")
         dev = advantages[0].device
         nmb, mbs = int(c0["num_minibatches"]), int(c0["minibatch_size"])
         batch_size = nmb * mbs
@@ -180,6 +211,11 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
         acc = torch.zeros((K, _lib.PPO_SCRATCH_BYTES // 8), dtype=torch.float64, device=dev)
         scratch = torch.empty(ops.ppo_grad_grouped_scratch_bytes(K, mbs), dtype=torch.uint8, device=dev)
         coefs = torch.tensor(coef_rows, dtype=torch.float32).to(dev)
+        anchor = {}
+        if anchor_logits is not None:
+            flat_anchor = [_flat_anchor(a, batch_size) for a in anchor_logits]  # alive until the update returns
+            anchor = dict(anchor_logits=torch.tensor([a.data_ptr() for a in flat_anchor], dtype=torch.int64).to(dev),
+                          kl_coef=torch.tensor(kl_coefs, dtype=torch.float32).to(dev))
 
         for epoch in range(n_epochs):
             perms = []
@@ -193,13 +229,15 @@ def make_population_update_step(configs, actor_forward_pass, optimizers, permuta
             tables = tables.pin_memory().to(dev, non_blocking=True)
             for mb in range(nmb):
                 ops.ppo_grad_grouped(tables[mb], coefs, blob, scratch, flat_g, stats_all[epoch, mb], acc, batch=mbs,
-                                     obs_dtype=obs_dtype, illegal_stat=stat_mode == "all" or mb == nmb - 1, tune=tune, **flags)
+                                     obs_dtype=obs_dtype, illegal_stat=stat_mode == "all" or mb == nmb - 1, tune=tune, **flags,
+                                     **anchor)
                 states = update_mlp_grouped_(optimizers, flat_p, flat_g, m, v, states, acc, blob)
 
-        out = []
+        results = []
         for k in range(K):
             env_state, last_obs, terminated_count = rest[k]
-            out.append(((new_params[k], states[k], env_state, last_obs, terminated_count, rngs[k]), _loss_info(stats_all[:, :, k])))
-        return out
+            results.append(((new_params[k], states[k], env_state, last_obs, terminated_count, rngs[k]), _loss_info(stats_all[:, :, k])))
+        out["anchor_kl"] = [stats_all[:, :, k, 7] for k in range(K)] if anchor else None
+        return results
 
-    return update_step
+    return WithOutputs(update_step, out)

@@ -15,6 +15,26 @@ from . import random as brandom
 from .env import BridgeBidding, State
 
 
+class WithOutputs:
+    """A callable plus outputs it leaves beside its return value, read as attributes (`roll_out.anchor_logits`,
+    `update_step.anchor_kl`): `fn` writes them into the dict `out`.  The function does not refer to the object that
+    exposes them, so a roll-out or update step is freed by reference counting when its last user drops it -- a reference
+    cycle would leave its CUDA graphs to the garbage collector, which may run inside another graph's capture."""
+    __slots__ = ("_fn", "_out")
+
+    def __init__(self, fn, out: dict):
+        self._fn, self._out = fn, out
+
+    def __call__(self, *args, **kwargs):
+        return self._fn(*args, **kwargs)
+
+    def __getattr__(self, name):
+        try:
+            return self._out[name]
+        except KeyError:
+            raise AttributeError(name) from None
+
+
 class _AutoResetStep:
     def __init__(self, env: BridgeBidding):
         self.env = env

@@ -54,6 +54,7 @@
  *   brl_mlp_pack_train    flat fp32 params -> device layout for brl_ppo_grad
  *   brl_mlp_adam_step     optimizer.update + apply_updates + refresh of that layout, one pass   src/update.py:168-169
  *   brl_ppo_grad_grouped / brl_mlp_adam_step_grouped   the two above for K learners at once (population training)
+ *   brl_ppo_grad_anchored / brl_ppo_grad_grouped_anchored   brl_ppo_grad(_grouped) + a KL penalty toward a fixed anchor policy
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -416,7 +417,7 @@ typedef struct BrlAdamParams {
  *          [5] in f32 old_log_prob[total]  [6] in f32 old_value[total]  [7] in f32 advantages[total]
  *          [8] in f32 targets[total]  [9] out f32 dlogits[B,38]  [10] out f32 dvalue[B]
  *          [11] out f32 stats[8] = {total_loss, value_loss, loss_actor, entropy, approx_kl, clipfracs,
- *               illegal_action_loss, 0}  [12] scratch, BRL_PPO_SCRATCH_BYTES, 16-byte aligned (f64[16] accumulators, then the
+ *               illegal_action_loss, 0 (the anchor KL of brl_ppo_grad_anchored)}  [12] scratch, BRL_PPO_SCRATCH_BYTES, 16-byte aligned (f64[16] accumulators, then the
  *               38 x 38 Gram partials of the illegal-probability matrix: illegal_action_loss is its SPECTRAL norm / 2,
  *               jnp.linalg.norm(X, ord=2) of a 2-D array, src/update.py:141-142) */
 int32_t brl_ppo_loss(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
@@ -463,6 +464,15 @@ int32_t brl_mlp_adam_step(brl_stream_t, void **buffers, const void *opaque, size
  *          [11] out f32 stats[8] (as brl_ppo_loss)  [12] scratch, BRL_PPO_SCRATCH_BYTES (as brl_ppo_loss); on return its f64
  *               element 14 = sum of squares of grads (the input of brl_adam_apply) */
 int32_t brl_ppo_grad(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_ppo_grad with a KL penalty toward a fixed anchor policy: the loss gains kl_coef * mean_b KL(pi(.|s_b) || alpha(.|s_b)),
+ * pi the policy distribution of the loss (masked softmax, or the unmasked one with BRL_PPO_UNMASKED_POLICY), alpha the
+ * softmax of the anchor's logits over the same action set (0 log 0 := 0).  d / d logit_j = kl_coef / B * pi_j (log pi_j -
+ * log alpha_j - KL_b) on the set, 0 elsewhere.  opaque = BrlPpoParams.
+ * buffers: [0..12] as brl_ppo_grad  [13] in f32 anchor_logits[total, 38] (the anchor net's logits for each trajectory row)
+ *          [14] in f32 kl_coef[1] (device scalar)
+ * stats[0] includes kl_coef * KL, stats[7] = mean_b KL_b.  With kl_coef = 0 the gradient and stats[0..6] are bit-equal to
+ * brl_ppo_grad's.  An empty batch (batch = 0) is a no-op and its buffers may be NULL. */
+int32_t brl_ppo_grad_anchored(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
 /* ---- population training: one optimizer step of K learners in the launches of one ------------------------------------
  * K PPO learners of the same shape (minibatch size B, flags) each take their step on their own weights, trajectory and
@@ -494,6 +504,11 @@ int64_t brl_ppo_grad_grouped_scratch_bytes(int64_t n_learners, int64_t batch);
  * Buffers [2], [3], [4] and [6] are 16-byte aligned.  Undefined: a table address that is not a valid buffer of the size
  * above, an index outside [0, total_k), buffers that overlap. */
 int32_t brl_ppo_grad_grouped(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_ppo_grad_anchored for K learners.  opaque = BrlPpoGroupedParams.
+ * buffers: [0..6] as brl_ppo_grad_grouped  [7] in i64 anchor_logits[K]: device address of learner k's f32 anchor logits
+ *          [total_k, 38]  [8] in f32 kl_coef[K]
+ * Learner k's results are bit-identical to a brl_ppo_grad_anchored call with its inputs.  An empty batch is a no-op. */
+int32_t brl_ppo_grad_grouped_anchored(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 /* brl_mlp_adam_step for K learners in one launch.  opaque = BrlAdamParams[K] (opaque_len = K * sizeof, 0 = no-op): learner
  * k's step count, learning rate, betas, eps and max_grad_norm; n = brl_mlp_num_params() for every k.
  * buffers: [0] inout f32 params[K, s]  [1] in f32 grads[K, s]  [2] inout f32 m[K, s]  [3] inout f32 v[K, s], s =
@@ -613,6 +628,8 @@ void brl_mlp_pack_train_xla(brl_stream_t, void **buffers, const char *opaque, si
 void brl_mlp_adam_step_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_ppo_grad_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_ppo_grad_anchored_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_ppo_grad_grouped_anchored_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_mlp_adam_step_grouped_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_act_log_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_eval_summary_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
