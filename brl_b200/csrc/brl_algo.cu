@@ -1,6 +1,7 @@
 // brl_algo.cu -- the small per-env algorithms around the environment: GAE reverse
 // scan, masked categorical (mode / Gumbel-argmax sample / log-prob), IMP reward,
-// match-statistic partial sums, transition reward gather.  sm_100a only.
+// match-statistic partial sums, transition reward gather, double-dummy par (its reward gather and match
+// statistics).  sm_100a only.
 #include <math.h>
 
 #include "common.h"
@@ -329,6 +330,89 @@ __global__ void __launch_bounds__(256) k_gather_reward(const float* __restrict__
     }
 }
 
+// ---- double-dummy par of each env's board (par_score), in the rewards layout by player id ------------------------------
+// Only the A word (dealer, vulnerability, seating) and the deal index of the packed state are read.
+__global__ void __launch_bounds__(256) k_par(const uint4* __restrict__ state, int64_t stride, const uint8_t* __restrict__ table,
+                                             float4* __restrict__ par, int32_t* __restrict__ contract, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    Env e;
+    e.A = state[3 * stride + i].z;
+    e.deal = state[4 * stride + i].w;
+    const Par p = par_score(e, TableRows{table});
+    const float v = (float)((f_player_at(e, 0u) >> 1) == 0u ? p.ns : -p.ns);  // par of the team of player ids {0, 1}
+    par[i] = make_float4(v, v, -v, -v);
+    if (contract != nullptr) contract[i] = p.contract;
+}
+
+// bidding against par over the two tables of a duplicate match, for the team of player ids {0, 1}: per table the IMPs of its
+// score against par and whether its final contract is the par contract (level, strain and declaring side; doubles ignored;
+// two passed-out boards match).  Table B has table A's board with the teams' seats swapped (env_duplicate_init), so its par
+// by player id is table A's negated.  sums[0..4] += {tables, sum imp, sum imp^2, sum |imp|, #par contract} in double.
+__device__ __forceinline__ bool reached_par(uint32_t seating, int32_t last_bid, int32_t last_bidder, int32_t par_contract) {
+    if (last_bid < 0 || par_contract < 0) return last_bid < 0 && par_contract < 0;
+    uint32_t side = 0u;  // the side of the seat the last bidder sits in
+#pragma unroll
+    for (uint32_t s = 0; s < 4u; ++s)
+        if (((seating >> (2u * s)) & 3u) == (uint32_t)last_bidder) side = s & 1u;
+    return last_bid == (par_contract & 0xFF) && side == ((uint32_t)par_contract >> 8 & 1u);
+}
+
+__global__ void __launch_bounds__(256) k_par_stats(const uint4* __restrict__ state, int64_t stride, const uint8_t* __restrict__ table,
+                                                   const float* __restrict__ rew_a, const int32_t* __restrict__ bid_a,
+                                                   const int32_t* __restrict__ bidder_a, const float* __restrict__ rew_b,
+                                                   const int32_t* __restrict__ bid_b, const int32_t* __restrict__ bidder_b,
+                                                   double* __restrict__ sums, int64_t n) {
+    double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        Env e;
+        e.A = state[3 * stride + i].z;
+        e.deal = state[4 * stride + i].w;
+        const Par p = par_score(e, TableRows{table});
+        const uint32_t s_a = f_seating(e);
+        const uint32_t s_b = (s_a >> 2 & 3u) | (s_a & 3u) << 2 | (s_a >> 6 & 3u) << 4 | (s_a >> 4 & 3u) << 6;  // env_duplicate_init
+        const float par_a = (float)((s_a & 3u) >> 1 == 0u ? p.ns : -p.ns);  // par of player ids {0, 1} at table A
+        const float imp_a = imp_of_difference(rew_a[4 * i] - par_a), imp_b = imp_of_difference(rew_b[4 * i] + par_a);
+        acc[0] += 2.0;
+        acc[1] += (double)imp_a + (double)imp_b;
+        acc[2] += (double)imp_a * imp_a + (double)imp_b * imp_b;
+        acc[3] += (double)fabsf(imp_a) + (double)fabsf(imp_b);
+        acc[4] += (reached_par(s_a, bid_a[i], bidder_a[i], p.contract) ? 1.0 : 0.0) +
+                  (reached_par(s_b, bid_b[i], bidder_b[i], p.contract) ? 1.0 : 0.0);
+    }
+    __shared__ double sh[5][8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+        if (lane == 0) sh[k][warp] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < 5) {
+        double t = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += sh[threadIdx.x][w];
+        if (t != 0.0) atomicAdd(&sums[threadIdx.x], t);
+    }
+}
+
+// k_gather_reward's par counterpart: a finished board's reward is IMP(score - par) / 24 from the actor's side
+__global__ void __launch_bounds__(256) k_gather_reward_par(const float* __restrict__ rewards, const int8_t* __restrict__ actor,
+                                                           const float* __restrict__ par, const uint8_t* __restrict__ done,
+                                                           float* __restrict__ out, int64_t n,
+                                                           unsigned long long* __restrict__ count) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool d = i < n && done[i] != 0;
+    if (i < n) {
+        const int64_t k = 4 * i + (actor[i] & 3);
+        out[i] = d ? imp_of_difference(rewards[k] - par[k]) / 24.0f : 0.0f;
+    }
+    if (count != nullptr) {
+        const int c = __syncthreads_count(d);
+        if (threadIdx.x == 0 && c > 0) atomicAdd(count, (unsigned long long)c);
+    }
+}
+
 
 int32_t launch_categorical(cudaStream_t stream, const float* logits, const unsigned char* mask, int32_t* action, float* log_prob,
                            int64_t n, int sample, uint64_t seed, int64_t env_offset, uint32_t step, const int32_t* row_index, float* logits_by_env) {
@@ -483,6 +567,58 @@ int32_t brl_gather_reward(brl_stream_t stream, void** b, const void* opaque, siz
         p->gamma, counting ? static_cast<const uint8_t*>(b[3]) : nullptr,
         counting ? static_cast<unsigned long long*>(b[4]) : nullptr);
     return check_launch("brl_gather_reward");
+}
+
+int32_t brl_par(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    static const char* names[] = {"state", "deal_table", "par", "contract"};
+    if ((rc = check_buffers("brl_par", b, names, 4, 1u << 3, 1u << 0 | 1u << 2)) != BRL_OK) return rc;
+    if ((reinterpret_cast<uintptr_t>(b[3]) & 3u) != 0) return fail(BRL_E_BUFFER, "brl_par: buffer 'contract' is not 4-byte aligned");
+    const int64_t stride = p->state_stride > 0 ? p->state_stride : p->n_envs;
+    if (stride < p->n_envs) return fail(BRL_E_OPAQUE, "brl_par: state_stride < n_envs");
+    k_par<<<(unsigned)((p->n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint4*>(b[0]), stride, static_cast<const uint8_t*>(b[1]), static_cast<float4*>(b[2]),
+        static_cast<int32_t*>(b[3]), p->n_envs);
+    return check_launch("brl_par");
+}
+
+int32_t brl_gather_reward_par(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    static const char* names[] = {"rewards", "actor", "par", "done", "reward", "count"};
+    const bool counting = (p->flags & BRL_F_COUNT_DONE) != 0;
+    if ((rc = check_buffers("brl_gather_reward_par", b, names, 6, counting ? 0u : 1u << 5, 1u << 0 | 1u << 2)) != BRL_OK) return rc;
+    if (counting && (reinterpret_cast<uintptr_t>(b[5]) & 7u) != 0)
+        return fail(BRL_E_BUFFER, "brl_gather_reward_par: buffer 'count' is not 8-byte aligned");
+    k_gather_reward_par<<<(unsigned)((p->n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const float*>(b[0]), static_cast<const int8_t*>(b[1]), static_cast<const float*>(b[2]),
+        static_cast<const uint8_t*>(b[3]), static_cast<float*>(b[4]), p->n_envs,
+        counting ? static_cast<unsigned long long*>(b[5]) : nullptr);
+    return check_launch("brl_gather_reward_par");
+}
+
+int32_t brl_par_stats(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    static const char* names[] = {"state", "deal_table", "rewards_a", "last_bid_a", "last_bidder_a", "rewards_b", "last_bid_b",
+                                  "last_bidder_b", "sums"};
+    if ((rc = check_buffers("brl_par_stats", b, names, 9, 0u, 1u << 0 | 1u << 2 | 1u << 5 | 1u << 8)) != BRL_OK) return rc;
+    const int64_t stride = p->state_stride > 0 ? p->state_stride : p->n_envs;
+    if (stride < p->n_envs) return fail(BRL_E_OPAQUE, "brl_par_stats: state_stride < n_envs");
+    unsigned grid = (unsigned)((p->n_envs + 255) / 256);
+    if (grid > 148u * 4u) grid = 148u * 4u;
+    k_par_stats<<<grid, 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint4*>(b[0]), stride, static_cast<const uint8_t*>(b[1]), static_cast<const float*>(b[2]),
+        static_cast<const int32_t*>(b[3]), static_cast<const int32_t*>(b[4]), static_cast<const float*>(b[5]),
+        static_cast<const int32_t*>(b[6]), static_cast<const int32_t*>(b[7]), static_cast<double*>(b[8]), p->n_envs);
+    return check_launch("brl_par_stats");
 }
 
 }  // extern "C"

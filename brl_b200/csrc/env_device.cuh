@@ -222,6 +222,80 @@ __device__ __forceinline__ float imp_of_difference(float d) {
     return d >= 0.0f ? (float)imp : -(float)imp;
 }
 
+// ---- double-dummy par (not in the reference; DESIGN.md f13, restated by tests/par_ref.py) ----------------------------
+// Par is the minimax value of this game over the deal's DD table t[seat][strain]:
+//   - side o (NS = seats 0/2, EW = 1/3) declaring bid c scores, with T the tricks of its declarer (the partner with more
+//     tricks in the strain; on a tie the one who comes first in the auction from the dealer),
+//     contract_score(c, undoubled, vul_o, T) when T >= level + 6 and contract_score(c, doubled, vul_o, T) otherwise;
+//     the NS score is that value for o = NS and its negative for o = EW;
+//   - the sides alternate, the dealer's side first.  With no contract the side to move passes or names any contract, and
+//     two passes with no contract pass the board out (0).  When o owns c the other side passes (the game ends at c) or
+//     names a contract c' > c, which makes it the owner with o to move;
+//   - NS maximises and EW minimises the NS score.
+// The par contract ends the line on which every side to move takes, among its best options, pass if it is one of them and
+// otherwise the lowest contract.  It is -1 when passed out, else bid | declarer_seat << 8 | doubled << 10.  This is a
+// definition of this project: no DDS par solver is involved, and the declarer rule is a simplification.
+struct Par {
+    int32_t ns;        // par in NS points
+    int32_t contract;  // par contract code
+};
+
+template <class Rows>
+__device__ __forceinline__ Par par_score(const Env& e, const Rows& rows) {
+    const uint32_t dealer = f_dealer(e);
+    int32_t tr[2][5];
+    uint32_t decl[2][5];
+#pragma unroll
+    for (uint32_t o = 0; o < 2u; ++o) {
+        const bool o_first = ((o - dealer) & 3u) < ((o + 2u - dealer) & 3u);
+#pragma unroll
+        for (uint32_t s = 0; s < 5u; ++s) {
+            const int32_t a = rows.tricks(e.deal, o, s), b = rows.tricks(e.deal, o + 2u, s);
+            const bool pick_a = a > b || (a == b && o_first);
+            tr[o][s] = pick_a ? a : b;
+            decl[o][s] = pick_a ? o : o + 2u;
+        }
+    }
+    const uint32_t vul[2] = {f_vul_ns(e), f_vul_ew(e)};
+    auto value = [&](uint32_t o, uint32_t c) {
+        const int32_t t = tr[o][c % 5u];
+        const int32_t s = contract_score(c, t < (int32_t)(c / 5u) + 7 ? 1u : 0u, 0u, vul[o], t);
+        return o == 0u ? s : -s;
+    };
+    // backward induction: V[o][c] = the value when o owns c and the other side m is to move, the better for m of passing
+    // and best[m] (m's optimum over its contracts above c)
+    int32_t V[2][35];
+    int32_t best[2] = {INT32_MIN, INT32_MAX};  // NS maximises, EW minimises
+    for (int c = 34; c >= 0; --c) {
+        const int32_t v0 = min(value(0u, (uint32_t)c), best[1]);
+        const int32_t v1 = max(value(1u, (uint32_t)c), best[0]);
+        V[0][c] = v0;
+        V[1][c] = v1;
+        best[0] = max(best[0], v0);
+        best[1] = min(best[1], v1);
+    }
+    const uint32_t d = dealer & 1u;
+    auto opt = [](uint32_t side, int32_t a, int32_t b) { return side == 0u ? max(a, b) : min(a, b); };
+    const int32_t after_pass = opt(d ^ 1u, 0, best[d ^ 1u]);  // the dealer's side passed: the other side's choice
+    const int32_t root = opt(d, after_pass, best[d]);
+    // the par line: pass when it is among the best options, else the lowest best contract
+    int owner = -1, c = -1;
+    int32_t target = root;
+    if (after_pass != root) owner = (int)d;
+    else if (after_pass != 0) owner = (int)(d ^ 1u), target = after_pass;
+    while (owner >= 0) {
+        int k = c + 1;
+        while (V[owner][k] != target) ++k;  // a best option exists: target is the optimum over these contracts
+        c = k;
+        if (value((uint32_t)owner, (uint32_t)c) == target) break;  // the other side passes
+        owner ^= 1;
+    }
+    if (owner < 0) return Par{0, -1};
+    const uint32_t strain = (uint32_t)c % 5u;
+    const uint32_t doubled = tr[owner][strain] < c / 5 + 7 ? 1u : 0u;
+    return Par{root, c | (int32_t)(decl[owner][strain] << 8) | (int32_t)(doubled << 10)};
+}
+
 __device__ __forceinline__ void history_set_bit(Env& e, uint32_t bit) {
     uint32_t w = bit >> 5, m = 1u << (bit & 31u);
 #pragma unroll

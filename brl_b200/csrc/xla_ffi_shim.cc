@@ -80,6 +80,9 @@
     X(brl_mlp_adam_step_grouped, "xixxix") \
     X(brl_ppo_grad_anchored, "iisiiiiiiioosii") \
     X(brl_ppo_grad_grouped_anchored, "iiisoosii") \
+    X(brl_par, "iioo") \
+    X(brl_gather_reward_par, "iiiiox") \
+    X(brl_par_stats, "iiiiiiiix") \
     /* end */
 
 namespace {

@@ -182,6 +182,15 @@ class BridgeBidding:
         ops.observe(state._packed, self.table, obs, None if player_id is None else player_id.to(torch.int8))
         return obs
 
+    def par(self, state: State):
+        """Double-dummy par of each env's board (DESIGN.md f13) -> (par f32[n, 4] by player id, as `rewards` is laid out,
+        contract i32[n]: -1 passed out, else bid | declarer_seat << 8 | doubled << 10)."""
+        n = state.num_envs
+        par = torch.empty((n, 4), dtype=torch.float32, device=self.device)
+        contract = torch.empty(n, dtype=torch.int32, device=self.device)
+        ops.par(state._packed, self.table, par, contract)
+        return par, contract
+
 
 def act_randomly(seed: int, state: State, step_index: int = 0, env_offset: int = 0) -> torch.Tensor:
     """`pgx.experimental.utils.act_randomly(key, state)` (src/duplicate.py:7,234): a uniform

@@ -653,6 +653,23 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
     return fn
 
 
+def par_statistics(eval_env, init_state, table_a_info, table_b_info) -> dict:
+    """Bidding against the double-dummy par (DESIGN.md f13) in a duplicate match, from the match's initial state (table A's)
+    and the two Table_infos a duplicate evaluator returned, for the team of player ids {0, 1} over the 2n tables:
+    `imp_vs_par` (mean, standard error) of IMP(score - par) -- the other team's is its exact negative --, `abs_imp_vs_par`
+    the mean |IMP vs par| and `par_contract_rate` the fraction of tables whose final contract is the par contract in level,
+    strain and declaring side (doubles ignored; two passed-out boards match).  One brl_par_stats kernel forms the f64 sums and
+    one all-reduce adds them over the ranks, so the result does not depend on the rank count."""
+    sums = torch.zeros(8, dtype=torch.float64, device=eval_env.device)
+    a, b = table_a_info, table_b_info
+    ops.par_stats(init_state._packed, eval_env.table, a.rewards, a.last_bid, a.last_bidder, b.rewards, b.last_bid, b.last_bidder,
+                  sums)
+    bdist.allreduce_sums(sums)
+    s = sums.cpu().numpy()
+    mean, se, _ = bdist.stats_from_sums((s[0], s[1], s[2], 0.0))
+    return {"imp_vs_par": (mean, se), "abs_imp_vs_par": s[3] / s[0], "par_contract_rate": s[4] / s[0]}
+
+
 def make_device_simple_evaluate(eval_env, team1_activation, team1_model_type, team2_activation, team2_model_type,
                                 team2_model_path, num_eval_envs, team2_params=None, *, tune: int = 0):
     """make_simple_evaluate (src/evaluation.py:11-66) as one brl_evaluate_match call: the same keys and per-env returns R, and

@@ -238,6 +238,32 @@ def gather_reward(rewards, actor, out, scale: float, done: Optional[torch.Tensor
           _params(rewards.shape[0], gamma=scale, flags=_lib.F_COUNT_DONE if counting else 0))
 
 
+def par(state_packed, table, out, contract: Optional[torch.Tensor] = None) -> None:
+    """Double-dummy par of each env's board (DESIGN.md f13): `out` f32[n, 4] in the rewards layout, by player id
+    (p, p, -p, -p) with p the par of the team of player ids {0, 1}; `contract` i32[n]: -1 when passed out, else
+    bid | declarer_seat << 8 | doubled << 10."""
+    n = state_packed.shape[1]
+    _call("brl_par", [_ptr(state_packed), _ptr(table), _ptr(out), _ptr(contract)],
+          _params(n, stride=state_packed.shape[1], n_deals=table.shape[0]))
+
+
+def par_stats(state_packed, table, rewards_a, last_bid_a, last_bidder_a, rewards_b, last_bid_b, last_bidder_b,
+              sums: torch.Tensor) -> None:
+    """sums f64[8] += {tables, sum IMP vs par, sum IMP^2, sum |IMP|, #par contract reached} of a duplicate match for the team
+    of player ids {0, 1}; `state_packed` is table A's initial state, the rest the two tables' Table_info fields."""
+    n = state_packed.shape[1]
+    _call("brl_par_stats", [_ptr(state_packed), _ptr(table), _ptr(rewards_a), _ptr(last_bid_a), _ptr(last_bidder_a),
+                            _ptr(rewards_b), _ptr(last_bid_b), _ptr(last_bidder_b), _ptr(sums)],
+          _params(n, stride=state_packed.shape[1], n_deals=table.shape[0]))
+
+
+def gather_reward_par(rewards, actor, par, done, out, count: Optional[torch.Tensor] = None) -> None:
+    """reward = done ? IMP(rewards[actor] - par[actor]) / 24 : 0, with `par` from `par` on the state before the step;
+    with `count` (int64[1]): count += sum(done) in the same launch."""
+    _call("brl_gather_reward_par", [_ptr(rewards), _ptr(actor), _ptr(par), _ptr(done), _ptr(out), _ptr(count)],
+          _params(rewards.shape[0], flags=_lib.F_COUNT_DONE if count is not None else 0))
+
+
 def mlp_pack(weights, biases, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Six haiku-layout fp32 (w[in,out], b[out]) pairs -> the packed bf16 hi/lo parameter blob (`out`: re-pack in place)."""
     dev = weights[0].device

@@ -7,6 +7,11 @@ run starts from) and `anchor_kl_coef` the weight of coef * mean KL(policy || anc
 roll-out records the anchor's logits, the update adds the term (a loss term: rewards, GAE and value targets are
 unchanged), and the log gains `train/anchor_kl`.  Unset (the default), every code path is the one without the feature.
 
+Double-dummy par (not in the reference; DESIGN.md f13): `reward_mode="par_imp"` trains on IMP(score - par) / 24 instead of
+score / reward_scale (roll_out.py), and `log_par=True` adds eval/imp_vs_par, eval/abs_imp_vs_par and eval/par_contract_rate
+of the eval/* duplicate match to the iterations that play it (evaluation.par_statistics).  The defaults ("score", False)
+leave every code path as it was.
+
 Everything heavy runs in the kernels behind `brl_b200.ops`; this file is the control
 plane only (config defaults, opponent selection, table rotation, logging hooks).  wandb,
 OmegaConf and the dataset download are out of scope (SURVEY 2): `log_fn` receives the same
@@ -30,12 +35,12 @@ from . import pbt as _pbt
 from . import random as brandom
 from .env import BridgeBidding
 from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_pfsp_probe,
-                         make_device_simple_evaluate, make_evaluate_log)
+                         make_device_simple_evaluate, make_evaluate_log, par_statistics)
 from .gae import make_calc_gae
 from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
 from .optim import OptState, make_optimizer
 from .pbt import default_pbt_config  # noqa: F401 -- ppo.default_pbt_config(): the options of train_population's `pbt`
-from .roll_out import make_roll_out
+from .roll_out import check_reward_mode, make_roll_out
 from .update import check_population_configs, make_population_update_step, make_update_step
 from .zoo import ModelZoo, device_zoo_fits
 
@@ -54,7 +59,8 @@ def default_config() -> dict:
         num_prioritized_envs=100, gamma=1.0, gae_lambda=0.95, clip_eps=0.2, ent_coef=0.001, vf_coef=0.5,
         value_clipping=True, global_gradient_clipping=True, anneal_lr=False, reward_scaling=False, max_grad_norm=0.5,
         reward_scale=7600.0, actor_illegal_action_mask=True, actor_illegal_action_penalty=False,
-        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0, anchor_model_path=None, anchor_kl_coef=0.0)
+        illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0, anchor_model_path=None, anchor_kl_coef=0.0,
+        reward_mode="score", log_par=False)
 
 
 def check_anchor_config(config: dict) -> None:
@@ -116,6 +122,7 @@ class Learner:
         make_fp = forward_pass_factory or make_forward_pass
         self.config = config = full_config(config)
         check_anchor_config(config)
+        check_reward_mode(config)
         self.log_fn = log_fn
         self.np_rng = np_rng or np.random.default_rng(config["seed"])
         self.dev = dev = torch.device(device)
@@ -221,8 +228,14 @@ class Learner:
         self.R = self.simple_evaluate(runner_state[0], eval_rng)                                  # ppo.py:365-368
         self.eval_log = {}
         if i % config["num_eval_step"] == 0:                                                      # ppo.py:369-374
-            log_info, _, _ = self.duplicate_evaluate(runner_state[0], eval_rng)
+            log_info, table_a_info, table_b_info = self.duplicate_evaluate(runner_state[0], eval_rng)
             self.eval_log = make_evaluate_log(log_info)
+            if config["log_par"]:  # the same match against par: its initial state from the keys it was played from
+                init_state = self.eval_env.init(self.duplicate_evaluate.buffers.keys)
+                par = par_statistics(self.eval_env, init_state, table_a_info, table_b_info)
+                self.eval_log.update({"eval/imp_vs_par": float(par["imp_vs_par"][0]),
+                                      "eval/abs_imp_vs_par": float(par["abs_imp_vs_par"]),
+                                      "eval/par_contract_rate": float(par["par_contract_rate"])})
         self.t_eval = time.time() - t0
 
         if config["self_play"]:                                                                   # ppo.py:376-470
@@ -386,6 +399,7 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
     check_population_configs(full)
     for c in full:
         check_anchor_config(c)
+        check_reward_mode(c)
     anchored = [bool(c["anchor_model_path"]) for c in full]
     if any(anchored) and not all(anchored):
         raise ValueError(f"population learners must all have a KL anchor or none: anchor_model_path is set for learners "

@@ -20,6 +20,12 @@ the anchor net on every step's observation (one `brl_mlp_forward` on the same bf
 `roll_out.anchor_logits[T, n, 38]`, which the update's KL term reads.  The buffer belongs to the roll-out and, like the
 trajectory, stays valid until the next call.  Anchored and plain calls keep separate buffers and CUDA graphs; the anchor
 is packed into its own fixed-address blob before an anchored replay.
+
+Reward (config["reward_mode"]): "score" (the default) is the reference's rewards[actor] / reward_scale.  "par_imp" takes a
+finished board's reward against its double-dummy par (DESIGN.md f13) instead: IMP(rewards[actor] - par[actor]) / 24.  Before
+each quad step `brl_par` writes the par of the state in `buf.packed` into the rollout's `par[n, 4]`: that state still holds
+the deal the quad step may finish, since auto-reset happens inside the step.  After the step `brl_gather_reward_par` replaces
+the reward gather.  Par mode is for competitive games with masked actors only (check_reward_mode).
 """
 from __future__ import annotations
 
@@ -35,6 +41,22 @@ from .utils import WithOutputs, auto_reset, single_play_step_free_run, single_pl
 
 _GRAPH_MIN_ENVS = 4096  # BRL_F_SEED_SALT lives in the fused forward launch
 _CAPTURE_KEY = 0x5EED    # host key the captured seeds are split from; the per-rollout key is the device salt
+REWARD_MODES = ("score", "par_imp")
+
+
+def check_reward_mode(config) -> None:
+    """ValueError for an unknown config["reward_mode"], and for "par_imp" in free-run games (the opponents never bid, so
+    competitive par is the wrong baseline) or without actor_illegal_action_mask (an illegal call ends a board with a
+    penalty, not a contract score)."""
+    mode = config.get("reward_mode", "score")
+    if mode not in REWARD_MODES:
+        raise ValueError(f"reward_mode must be one of {REWARD_MODES}; got {mode!r}")
+    if mode == "par_imp":
+        if config["game_mode"] == "free-run":
+            raise ValueError('reward_mode="par_imp" needs game_mode="competitive": in free-run the opponents never bid')
+        if not config["actor_illegal_action_mask"]:
+            raise ValueError('reward_mode="par_imp" needs actor_illegal_action_mask: an illegal call ends a board with a '
+                             'penalty, not a contract score')
 
 
 class Transition(NamedTuple):
@@ -51,7 +73,7 @@ class Transition(NamedTuple):
 class _Buffers:
     """Everything one rollout reads and writes, at fixed addresses."""
 
-    def __init__(self, T, n, dev, obs_dtype):
+    def __init__(self, T, n, dev, obs_dtype, par_mode=False):
         self.T, self.n = T, n
         self.done = torch.empty((T, n), dtype=torch.uint8, device=dev)
         self.action = torch.empty((T, n), dtype=torch.int32, device=dev)
@@ -65,6 +87,7 @@ class _Buffers:
         self.player = torch.empty((2, n), dtype=torch.int8, device=dev)                    # player to act, alternating per step
         self.term0 = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.count = torch.zeros(1, dtype=torch.int64, device=dev)
+        self.par = torch.empty((n, 4), dtype=torch.float32, device=dev) if par_mode else None  # par of the pre-step state
 
     def state(self, env, t):
         """State view whose outputs are the buffers step t writes (obs / mask slot t, done[t-1], player[t % 2])"""
@@ -99,10 +122,13 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
         make_step_fn = single_play_step_free_run
     else:
         raise ValueError(config["game_mode"])
+    check_reward_mode(config)
+    reward_mode = config.get("reward_mode", "score")
+    par_mode = reward_mode == "par_imp"
     T = int(config["num_steps"])
     scale = float(config["reward_scale"])
     obs_dtype = getattr(actor_forward_pass, "input_dtype", torch.float32)
-    cache = {}  # (n, anchored) -> dict(buf, graph, blobs, salt, anchor_logits, ...)
+    cache = {}  # (n, anchored, reward_mode) -> dict(buf, graph, blobs, salt, anchor_logits, ...)
     out = {"anchor_logits": None}
 
     def body(buf, params, opp_params, rng, trace, anchor=None):
@@ -119,10 +145,15 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
                 anchor_params, anchor_logits, anchor_value = anchor
                 anchor_forward_pass.forward_into(anchor_params, buf.obs[t], anchor_logits[t], anchor_value)
             rng, _rng = brandom.split(rng)
+            if par_mode:
+                ops.par(buf.packed, env.table, buf.par)
             cur = step_fn(cur, buf.action[t], _rng, out_state=buf.state(env, t + 1))                                # :84
             # reward = rewards[actor] / scale with actor = the player who was to act BEFORE the quad step (still in the
             # other player buffer), and terminated_count += sum(done)                                             :85-94
-            ops.gather_reward(buf.rewards, buf.player[t % 2], buf.reward[t], scale, done=buf.done[t], count=buf.count)
+            if par_mode:
+                ops.gather_reward_par(buf.rewards, buf.player[t % 2], buf.par, buf.done[t], buf.reward[t], count=buf.count)
+            else:
+                ops.gather_reward(buf.rewards, buf.player[t % 2], buf.reward[t], scale, done=buf.done[t], count=buf.count)
         return cur, rng
 
     def finish(buf, params, opt_state, cur, terminated_count, rng):
@@ -145,9 +176,9 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
             os.environ.get("BRL_ROLLOUT_GRAPH", "1") != "0" and \
             hasattr(actor_forward_pass, "pack_into") and hasattr(opp_forward_pass, "pack_into") and \
             (not anchored or hasattr(anchor_forward_pass, "pack_into"))  # tensor-core nets only
-        c = cache.get((n, anchored))
+        c = cache.get((n, anchored, reward_mode))
         if c is None:
-            c = cache[(n, anchored)] = {"buf": _Buffers(T, n, dev, obs_dtype), "graph": None}
+            c = cache[(n, anchored, reward_mode)] = {"buf": _Buffers(T, n, dev, obs_dtype, par_mode), "graph": None}
             if anchored:
                 c["anchor_logits"] = torch.empty((T, n, ops.NUM_ACTIONS), dtype=torch.float32, device=dev)
                 c["anchor_value"] = torch.empty(n, dtype=torch.float32, device=dev)

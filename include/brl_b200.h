@@ -55,6 +55,8 @@
  *   brl_mlp_adam_step     optimizer.update + apply_updates + refresh of that layout, one pass   src/update.py:168-169
  *   brl_ppo_grad_grouped / brl_mlp_adam_step_grouped   the two above for K learners at once (population training)
  *   brl_ppo_grad_anchored / brl_ppo_grad_grouped_anchored   brl_ppo_grad(_grouped) + a KL penalty toward a fixed anchor policy
+ *   brl_par / brl_gather_reward_par / brl_par_stats   not in the reference: the double-dummy par of each board, the
+ *                         transition reward as IMPs against it, and a duplicate match's bidding against it (DESIGN.md f13)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -232,6 +234,31 @@ int32_t brl_state_fields(brl_stream_t, void **buffers, const void *opaque, size_
  *          with BRL_F_COUNT_DONE: [3] in u8 done[n]  [4] inout u64 terminated_count[1] += sum(done)
  * scale passed in BrlParams.gamma. */
 int32_t brl_gather_reward(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
+/* Double-dummy par of each env's board (not in the reference; DESIGN.md f13 defines it): the minimax value of competitive
+ * bidding over the deal row's DD table, with the env's dealer and vulnerability.
+ * buffers: [0] in state (16-byte aligned)  [1] in deal_table
+ *          [2] out f32 par[n,4] (16-byte aligned) in the rewards layout: by player id (p, p, -p, -p), p = par of the
+ *              team of player ids {0, 1} under the state's seating
+ *          [3] out i32 contract[n] (NULL ok): -1 passed out, else bid | declarer_seat << 8 | doubled << 10 */
+int32_t brl_par(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
+/* brl_gather_reward against par: reward = done ? IMP(rewards[actor] - par[actor]) / 24 : 0 (24 = the largest IMP).
+ * buffers: [0] in f32 rewards[n,4]  [1] in i8 actor[n]  [2] in f32 par[n,4] (brl_par of the state before the step)
+ *          [3] in u8 done[n]  [4] out f32 reward[n]
+ *          [5] inout u64 terminated_count[1] += sum(done) -- read ONLY with BRL_F_COUNT_DONE (8-byte aligned)
+ * rewards and par 16-byte aligned. */
+int32_t brl_gather_reward_par(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
+/* Bidding against par over the two tables of a duplicate match (brl_evaluate_match's Table_infos), for the team of player
+ * ids {0, 1}: per table IMP(rewards[0] - par[0]), and whether the final contract is the par contract in level, strain and
+ * declaring side (doubles ignored; two passed-out boards match).  Table B is table A's board with the teams' seats swapped.
+ * buffers: [0] in state: table A's initial state (16-byte aligned)  [1] in deal_table
+ *          [2] in f32 rewards_a[n,4]  [3] in i32 last_bid_a[n]  [4] in i32 last_bidder_a[n]
+ *          [5] in f32 rewards_b[n,4]  [6] in i32 last_bid_b[n]  [7] in i32 last_bidder_b[n]
+ *          [8] inout f64 sums[8] += {tables, sum imp, sum imp^2, sum |imp|, #par contract, 0, 0, 0}
+ * rewards_a / rewards_b / sums 16-byte aligned.  The sums are integers: every order of addition gives the same result. */
+int32_t brl_par_stats(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
 /* ---- policy / value net on the tensor cores (src/models.py:23-33, "DeepMind" 4x1024 ReLU) ----
  * Weights are packed once (transposed to K-major bf16 hi/lo pairs); the forward is five
@@ -636,6 +663,9 @@ void brl_eval_summary_xla(brl_stream_t, void **buffers, const char *opaque, size
 void brl_sl_examples_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_sl_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_sl_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_gather_reward_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------
  * Host-buffer convenience layer (the call a non-JAX host makes): the library

@@ -8,9 +8,8 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the KL-anchored PPO loss head: k_ppo_loss gained a template argument pack (empty for the plain
-loss head, which cu++filt then prints as `k_ppo_loss<Args, >`), and the anchored instantiations k_ppo_loss<Args, PpoAnchor>
-are new.  Replace both tables for another change."""
+RENAMES and ADDED record the double-dummy par: no kernel is renamed, and k_par (brl_par), k_gather_reward_par
+(brl_gather_reward_par) and k_par_stats (brl_par_stats) are new.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -18,8 +17,8 @@ import subprocess
 import sys
 from collections import OrderedDict
 
-RENAMES = [(r"^brl::k_ppo_loss<(brl::Ppo(Group)?Args)>$", r"brl::k_ppo_loss<\1, >")]  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-ADDED = [r"^brl::k_ppo_loss<brl::Ppo(Group)?Args, brl::PpoAnchor>$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
+RENAMES = []  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
+ADDED = [r"^brl::k_par$", r"^brl::k_gather_reward_par$", r"^brl::k_par_stats$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):
