@@ -33,6 +33,7 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_mlp_num_params", "brl_mlp_train_blob_bytes", "brl_mlp_train_scratch_bytes", "brl_mlp_train_trace_offset",
         "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes",
         "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes",
+        "brl_evaluate_match_partner_scratch_bytes",
         "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
@@ -60,6 +61,8 @@ MATCH_OK, MATCH_BAD_MODEL, MATCH_STEP_BOUND = 0, 1, 2  # its status codes (BRL_M
 F_TUNE_MLP_LAYERS, F_TUNE_MLP_FUSED = 1 << 29, 1 << 30  # pin the policy forward's path (BRL_F_TUNE_MLP_*)
 EVAL_MATCH_DUPLICATE, EVAL_MATCH_SINGLE, EVAL_MATCH_SIMPLE = 1, 2, 3  # brl_evaluate_match's modes (BRL_EVAL_MATCH_*)
 F_EVAL_FREE_RUN = 0x0008  # brl_evaluate_match: team 2 always passes (BRL_F_EVAL_FREE_RUN)
+F_EVAL_PARTNER = 1 << 25  # brl_evaluate_match: a 3-net pool, net 2 the actor's partner (BRL_F_EVAL_PARTNER)
+F_PLAYER_MODELS = 1 << 24  # brl_model_rows / brl_duplicate_match: env_models[n, 4] by player id (BRL_F_PLAYER_MODELS)
 
 
 def f_eval_match(mode: int) -> int:

@@ -156,23 +156,26 @@ __global__ void __launch_bounds__(1024) k_team_rows(const int8_t* __restrict__ p
 
 // ---- live-env grouping by acting net over a pool (workspace/eval_selfplay_league.py) ---------------------------
 // k_team_rows for many matches at once: env i is played by net env_models[i][0] for players 0/1 and env_models[i][1] for
-// players 2/3 (src/evaluation.py:124-151).  Count per net, lay the nets' groups out padded to kGroupRows rows, scatter.  The
+// players 2/3 (src/evaluation.py:124-151); with BRL_F_PLAYER_MODELS (kStride 4) by net env_models[i][player] of each player.  Count per net, lay the nets' groups out padded to kGroupRows rows, scatter.  The
 // envs of one match are contiguous, so a warp nearly always holds one or two nets: one atomic per net and warp.
 // A live env whose acting net id is outside [0, M) invalidates the grouping: offsets[M] (the count the host reads anyway to
 // size the forward) becomes -1, so the error surfaces before any forward runs, without an extra host read.
 constexpr int kNotListed = -1, kBadModel = -2;
+template <int kStride>
 __device__ __forceinline__ int acting_model(const int8_t* player, const uint8_t* done, const int32_t* env_models, int64_t i,
                                             int64_t n, int n_models) {
+    static_assert(kStride == 2 || kStride == 4, "env_models holds a net per team or per player");
     if (i >= n || (done != nullptr && done[i] != 0)) return kNotListed;
-    const int m = env_models[2 * i + (player[i] < 2 ? 0 : 1)];
+    const int m = env_models[kStride * i + (kStride == 4 ? (player[i] & 3) : (player[i] < 2 ? 0 : 1))];
     return m >= 0 && m < n_models ? m : kBadModel;
 }
 
+template <int kStride>
 __global__ void __launch_bounds__(256) k_model_count(const int8_t* __restrict__ player, const uint8_t* __restrict__ done,
                                                      const int32_t* __restrict__ env_models, int32_t* __restrict__ counts,
                                                      int32_t* __restrict__ offsets, int64_t n, int n_models) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int m = acting_model(player, done, env_models, i, n, n_models);
+    const int m = acting_model<kStride>(player, done, env_models, i, n, n_models);
     const unsigned peers = __match_any_sync(0xffffffffu, m);
     if ((threadIdx.x & 31) != __ffs(peers) - 1) return;
     if (m >= 0) atomicAdd(&counts[m], __popc(peers));
@@ -229,12 +232,13 @@ __global__ void __launch_bounds__(1024) k_model_offsets(int32_t* __restrict__ co
     if (threadIdx.x == 0) offsets[n_models] = bad ? -1 : carry;
 }
 
+template <int kStride>
 __global__ void __launch_bounds__(256) k_model_scatter(const int8_t* __restrict__ player, const uint8_t* __restrict__ done,
                                                        const int32_t* __restrict__ env_models, const int32_t* __restrict__ offsets,
                                                        int32_t* __restrict__ cursor, int32_t* __restrict__ rows, int64_t n, int n_models) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
-    const int m = acting_model(player, done, env_models, i, n, n_models);
+    const int m = acting_model<kStride>(player, done, env_models, i, n, n_models);
     const unsigned peers = __match_any_sync(0xffffffffu, m);
     const int leader = __ffs(peers) - 1;
     int base = 0;
@@ -414,6 +418,21 @@ __global__ void __launch_bounds__(256) k_gather_reward_par(const float* __restri
 }
 
 
+// brl_model_rows' three kernels for env_models[n, kStride] (counts and offsets[M] already zeroed)
+template <int kStride>
+static void model_rows_launch(cudaStream_t s, void** b, int64_t n, int n_models) {
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    const int8_t* player = static_cast<const int8_t*>(b[0]);
+    const uint8_t* done = static_cast<const uint8_t*>(b[1]);
+    const int32_t* env_models = static_cast<const int32_t*>(b[2]);
+    int32_t* counts = static_cast<int32_t*>(b[4]);
+    k_model_count<kStride><<<grid, 256, 0, s>>>(player, done, env_models, counts, static_cast<int32_t*>(b[5]), n, n_models);
+    k_model_offsets<<<1, 1024, 0, s>>>(counts, static_cast<int32_t*>(b[5]), static_cast<int32_t*>(b[6]), static_cast<int32_t*>(b[3]),
+                                       n_models);
+    k_model_scatter<kStride><<<grid, 256, 0, s>>>(player, done, env_models, static_cast<const int32_t*>(b[5]), counts,
+                                                  static_cast<int32_t*>(b[3]), n, n_models);
+}
+
 int32_t launch_categorical(cudaStream_t stream, const float* logits, const unsigned char* mask, int32_t* action, float* log_prob,
                            int64_t n, int sample, uint64_t seed, int64_t env_offset, uint32_t step, const int32_t* row_index, float* logits_by_env) {
     unsigned grid = (unsigned)((n + 3) / 4);  // one warp per env row
@@ -541,15 +560,10 @@ int32_t brl_model_rows(brl_stream_t stream, void** b, const void* opaque, size_t
     if (cudaMemsetAsync(counts, 0, n_models * sizeof(int32_t), s) != cudaSuccess ||
         cudaMemsetAsync(static_cast<int32_t*>(b[5]) + n_models, 0, sizeof(int32_t), s) != cudaSuccess)
         return check_launch("brl_model_rows");
-    const unsigned grid = (unsigned)((p->n_envs + 255) / 256);
-    const int8_t* player = static_cast<const int8_t*>(b[0]);
-    const uint8_t* done = static_cast<const uint8_t*>(b[1]);
-    const int32_t* env_models = static_cast<const int32_t*>(b[2]);
-    k_model_count<<<grid, 256, 0, s>>>(player, done, env_models, counts, static_cast<int32_t*>(b[5]), p->n_envs, (int)n_models);
-    k_model_offsets<<<1, 1024, 0, s>>>(counts, static_cast<int32_t*>(b[5]), static_cast<int32_t*>(b[6]), static_cast<int32_t*>(b[3]),
-                                       (int)n_models);
-    k_model_scatter<<<grid, 256, 0, s>>>(player, done, env_models, static_cast<const int32_t*>(b[5]), counts,
-                                         static_cast<int32_t*>(b[3]), p->n_envs, (int)n_models);
+    if (p->flags & BRL_F_PLAYER_MODELS)
+        model_rows_launch<4>(s, b, p->n_envs, (int)n_models);
+    else
+        model_rows_launch<2>(s, b, p->n_envs, (int)n_models);
     return check_launch("brl_model_rows");
 }
 

@@ -44,6 +44,12 @@ __global__ void __launch_bounds__(256) k_pair_models(int32_t* __restrict__ env_m
     if (i < n) reinterpret_cast<int2*>(env_models)[i] = make_int2(0, 1);
 }
 
+// BRL_F_EVAL_PARTNER: every env's nets by player id (duplicate / single table: actor, partner, opponent, opponent)
+__global__ void __launch_bounds__(256) k_player_models(int32_t* __restrict__ env_models, int4 ids, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) reinterpret_cast<int4*>(env_models)[i] = ids;
+}
+
 __global__ void __launch_bounds__(256) k_add_reward(float* __restrict__ cum_return, const float4* __restrict__ rewards, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) cum_return[i] += rewards[i].x;  // cum_return += state.rewards[:, 0] (src/evaluation.py:167-169)
@@ -58,6 +64,17 @@ __global__ void __launch_bounds__(256) k_actor_models(int32_t* __restrict__ env_
     const int8_t p = player[i];
     actor[i] = p;
     reinterpret_cast<int2*>(env_models)[i] = p < 2 ? make_int2(0, 1) : make_int2(1, 0);
+}
+
+// k_actor_models with a partner, by player id: the initial player p plays net 0, its partner p ^ 1 net 2, the other team net 1
+__global__ void __launch_bounds__(256) k_actor_partner_models(int32_t* __restrict__ env_models, int8_t* __restrict__ actor,
+                                                              const int8_t* __restrict__ player, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int8_t p = player[i];
+    actor[i] = p;
+    const int own = p & 1 ? 2 : 0, other = 2 - own;  // player ids 0/1 and 2/3 are partners
+    reinterpret_cast<int4*>(env_models)[i] = p < 2 ? make_int4(own, other, 1, 1) : make_int4(1, 1, own, other);
 }
 
 __global__ void __launch_bounds__(256) k_add_actor_reward(float* __restrict__ R, const float* __restrict__ rewards,
@@ -110,7 +127,7 @@ struct MatchLayout {
         forward, logits, fields[6], rewards_sum, actor, total;
 };
 
-static MatchLayout match_layout(int64_t n, int64_t M, int mode = 0) {
+static MatchLayout match_layout(int64_t n, int64_t M, int mode = 0, bool player_models = false) {
     MatchLayout L{};
     size_t off = 0;
     auto take = [&](size_t bytes) {
@@ -134,7 +151,7 @@ static MatchLayout match_layout(int64_t n, int64_t M, int mode = 0) {
         L.info[t][4] = take(un);
         L.info[t][5] = take(un);
     }
-    L.env_models = take(un * 8);
+    L.env_models = take(un * (player_models ? 16 : 8));
     L.rows = take(cap * 4);
     L.counts = take((size_t)M * 4);
     L.offsets = take((size_t)(M + 1) * 4);
@@ -157,6 +174,8 @@ struct MatchPlan {
     const char* who;  // the op, for error messages
     int mode;         // 0: brl_duplicate_match; else BRL_EVAL_MATCH_*
     bool free_run;    // brl_evaluate_match: team 2 always passes
+    bool partner;     // brl_evaluate_match: BRL_F_EVAL_PARTNER
+    bool player_models;  // env_models[n, 4] by player id (BRL_F_PLAYER_MODELS)
     int64_t n, cap, P;
     int M;
     int32_t n_deals, flags;
@@ -210,6 +229,7 @@ static int32_t model_rows(const MatchPlan& q, cudaStream_t s) {
     void* b[7] = {q.player, q.terminated, q.env_models, q.at(q.L.rows), q.at(q.L.counts), q.offsets(), q.at(q.L.block_model)};
     BrlParams p = env_params(q, q.n);
     p.k_steps = q.M;
+    if (q.player_models) p.flags |= BRL_F_PLAYER_MODELS;
     return brl_model_rows(s, b, &p, sizeof(p));
 }
 
@@ -377,16 +397,23 @@ static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, 
         (q.acc && cudaMemsetAsync(q.acc, 0, un * BRL_EVAL_ACC_COLS * sizeof(float), s0) != cudaSuccess) ||
         (q.logits && cudaMemsetAsync(q.logits, 0, un * BRL_NUM_ACTIONS * sizeof(float), s0) != cudaSuccess) ||
         (q.rewards_sum && cudaMemsetAsync(q.rewards_sum, 0, un * 16, s0) != cudaSuccess) ||
-        (q.free_run && cudaMemsetAsync(q.env_models, 0, un * 8, s0) != cudaSuccess))  // free-run: net 0 forwards every row
+        (q.free_run && !q.partner && cudaMemsetAsync(q.env_models, 0, un * 8, s0) != cudaSuccess))  // free-run: net 0 forwards every row
         return launched(q.who, "memset");
-    if (q.default_models) k_pair_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.n);
+    if (q.partner && q.mode != BRL_EVAL_MATCH_SIMPLE)  // free-run: net 0 forwards team 2's rows, team 1's split between nets 0 / 2
+        k_player_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.free_run ? make_int4(0, 2, 0, 0) : make_int4(0, 2, 1, 1), q.n);
+    else if (q.default_models)
+        k_pair_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.n);
     // src/evaluation.py:93-95: the envs from the given keys, observation in bf16 (what the forward reads)
     void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
                    q.player};
     BrlParams p = env_params(q, q.n);
     if ((rc = brl_init(s0, bi, &p, sizeof(p)))) return rc;
     if (q.mode == BRL_EVAL_MATCH_SIMPLE) {
-        k_actor_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player), q.n);
+        if (q.partner)
+            k_actor_partner_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player),
+                                                                q.n);
+        else
+            k_actor_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player), q.n);
         if ((rc = launched(q.who, "actor"))) return rc;
     }
     if (q.mode == 0 || q.mode == BRL_EVAL_MATCH_DUPLICATE) {
@@ -491,7 +518,7 @@ static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p,
 }
 
 // the plan's fields every mode shares; the env buffers and Table_infos start in the scratch
-static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_t M, void* scratch) {
+static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_t M, void* scratch, bool player_models = false) {
     MatchPlan q{};
     q.who = who;
     q.mode = mode;
@@ -503,7 +530,8 @@ static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_
     q.illegal_penalty = p->illegal_penalty;
     q.illegal_bonus = p->illegal_bonus;
     q.scratch = static_cast<unsigned char*>(scratch);
-    q.L = match_layout(q.n, M, mode);
+    q.player_models = player_models;
+    q.L = match_layout(q.n, M, mode, player_models);
     for (int t = 0; t < 2; ++t)
         for (int k = 0; k < 6; ++k) q.info[t][k] = q.at(q.L.info[t][k]);
     q.state = q.at(q.L.state);
@@ -539,7 +567,10 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     if (!p) return rc;
     if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
     const int64_t M = p->k_steps, P = (int64_t)p->step;
+    const bool player_models = (p->flags & BRL_F_PLAYER_MODELS) != 0;
     if (M <= 0) return fail(BRL_E_OPAQUE, "brl_duplicate_match: k_steps (the pool's model count) must be > 0");
+    if (player_models && b[3] == nullptr)
+        return fail(BRL_E_BUFFER, "brl_duplicate_match: BRL_F_PLAYER_MODELS needs env_models [3] (i32[n, 4])");
     if (b[3] == nullptr && M != 2) return fail(BRL_E_OPAQUE, "brl_duplicate_match: without env_models the pool must hold 2 nets (got %lld)", (long long)M);
     if ((b[4] != nullptr) != (P > 0))
         return fail(BRL_E_OPAQUE, "brl_duplicate_match: step (the range count, %lld) must be > 0 exactly when the range offsets are given", (long long)P);
@@ -574,6 +605,7 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
         for (int t = 0; t < 2; ++t)
             for (int k = 0; k < 6; ++k) q.info[t][k] = b[9 + 6 * t + k];
     q.default_models = b[3] == nullptr;
+    q.player_models = player_models;  // the caller's env_models; the scratch keeps its [n, 2] layout
     if (!q.default_models) q.env_models = static_cast<int32_t*>(b[3]);
     return run_match(q, (cudaStream_t)stream, p, b, 21);
 }
@@ -581,6 +613,11 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
 int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode) {
     if (n_envs <= 0 || mode < BRL_EVAL_MATCH_DUPLICATE || mode > BRL_EVAL_MATCH_SIMPLE) return 0;
     return (int64_t)match_layout(n_envs, 2, (int)mode).total;
+}
+
+int64_t brl_evaluate_match_partner_scratch_bytes(int64_t n_envs, int64_t mode) {
+    if (n_envs <= 0 || mode < BRL_EVAL_MATCH_DUPLICATE || mode > BRL_EVAL_MATCH_SIMPLE) return 0;
+    return (int64_t)match_layout(n_envs, 3, (int)mode, true).total;
 }
 
 int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, size_t len) {
@@ -593,6 +630,9 @@ int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, si
     if (mode < BRL_EVAL_MATCH_DUPLICATE || mode > BRL_EVAL_MATCH_SIMPLE)
         return fail(BRL_E_OPAQUE, "brl_evaluate_match: flags name no mode (BRL_F_EVAL_MATCH(BRL_EVAL_MATCH_*))");
     if (free_run && !full) return fail(BRL_E_OPAQUE, "brl_evaluate_match: BRL_F_EVAL_FREE_RUN is a mode of the full-statistics evaluation");
+    const bool partner = (p->flags & BRL_F_EVAL_PARTNER) != 0;
+    if (partner && p->k_steps != 3)
+        return fail(BRL_E_OPAQUE, "brl_evaluate_match: BRL_F_EVAL_PARTNER needs a pool of 3 nets, k_steps = 3 (got %lld)", (long long)p->k_steps);
     if (p->n_envs > INT32_MAX / 2) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_envs too large");
     if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_deals must be > 0");
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_evaluate_match: sampling is not supported (argmax only)");
@@ -618,8 +658,9 @@ int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, si
             return fail(BRL_E_BUFFER, "brl_evaluate_match: the final state, observation or rewards are not 16-byte aligned (mask: 2)");
     }
 
-    MatchPlan q = base_plan("brl_evaluate_match", mode, p, 2, b[3]);
+    MatchPlan q = base_plan("brl_evaluate_match", mode, p, partner ? 3 : 2, b[3], partner);
     q.free_run = free_run;
+    q.partner = partner;
     q.keys = b[0];
     q.table = b[1];
     q.pool = static_cast<const unsigned char*>(b[2]);

@@ -37,6 +37,17 @@ class _TeamRows:
         return self.rows1[:c1], self.rows2[:c2]
 
 
+def _act_team(forward_pass, params, partner, state, action, rows, logits=None):
+    """the team of `rows` decides: `params` for all of them, or, with a `partner`, `params` for the team's first player
+    (player id 0 / 2) and `partner` for the second (1 / 3)"""
+    if partner is None:
+        forward_pass.act_rows(params, state.observation, state._mask_u8, action, rows, logits=logits)
+        return
+    second = (state.current_player[rows.long()] & 1).bool()
+    forward_pass.act_rows(params, state.observation, state._mask_u8, action, rows[~second], logits=logits)
+    forward_pass.act_rows(partner, state.observation, state._mask_u8, action, rows[second], logits=logits)
+
+
 def _bf16_state(env, keys):
     """env.init with the observation written directly in bf16 (the tensor-core nets' input dtype; the observation of
     these loops is read by the nets only)"""
@@ -54,12 +65,14 @@ def make_simple_evaluate(eval_env, team1_activation, team1_model_type, team2_act
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
     opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
 
-    def simple_evaluate(actor_params, rng, trace=None):
+    def simple_evaluate(actor_params, rng, trace=None, partner_params=None):
         """`trace` (a list, tests only) receives the four sub-step action tensors of every quad step and finally
-        ("R", per-env return) -- the inputs of an oracle replay."""
+        ("R", per-env return) -- the inputs of an oracle replay.  `partner_params`: the actor's partner (the quad step's
+        sub-step 3, of the actor's architecture) instead of the actor itself."""
         step_fn = single_play_step_two_policy_commpetitive_deterministic(
             step_fn=eval_env.step, actor_params=actor_params, actor_forward_pass=actor_forward_pass,
-            opp_params=opp_params, opp_forward_pass=opp_forward_pass)
+            opp_params=opp_params, opp_forward_pass=opp_forward_pass,
+            partner_forward_pass=actor_forward_pass if partner_params is not None else None, partner_params=partner_params)
         step_fn.trace = trace
         rng_key, sub_key = brandom.split(rng)
         state = eval_env.init(eval_env.make_keys(sub_key, num_eval_envs))
@@ -93,10 +106,13 @@ def make_simple_duplicate_evaluate(eval_env, team1_activation, team1_model_type,
     team1_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     team2_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
 
-    def duplicate_evaluate(team1_params, team2_params, rng_key, trace=None, record=None, local_sums=None):
+    def duplicate_evaluate(team1_params, team2_params, rng_key, trace=None, record=None, local_sums=None, team1_partner=None,
+                           team2_partner=None):
         """`record` (a list) receives per step (action, table_a.terminated, table_b.terminated) BEFORE the step --
         the input of board_log.match_to_board_logs.  `local_sums` (f64[8] tensor): accumulate this rank's partial
-        statistics there and skip the all-reduce (the league evaluator reduces all its matches at once)."""
+        statistics there and skip the all-reduce (the league evaluator reduces all its matches at once).
+        `team1_partner` / `team2_partner`: the net of player 1 / player 3 (of its team's architecture) instead of the team's
+        net, which then plays player 0 / 2 only -- a partnership of two nets (player ids keep their team at both tables)."""
         step_fn = duplicate_step(eval_env.step)
         rng_key, sub_key = brandom.split(rng_key)
         state = _bf16_state(eval_env, eval_env.make_keys(sub_key, num_eval_envs, env_offset))  # :93-95
@@ -111,8 +127,8 @@ def make_simple_duplicate_evaluate(eval_env, team1_activation, team1_model_type,
             rows1, rows2 = teams.split(state.current_player, state._terminated_u8)
             if rows1.shape[0] + rows2.shape[0] == 0:                                       # :120-122 ~terminated.all()
                 break
-            team1_forward_pass.act_rows(team1_params, state.observation, state._mask_u8, action, rows1)
-            team2_forward_pass.act_rows(team2_params, state.observation, state._mask_u8, action, rows2)
+            _act_team(team1_forward_pass, team1_params, team1_partner, state, action, rows1)
+            _act_team(team2_forward_pass, team2_params, team2_partner, state, action, rows2)
             if trace is not None:  # tests replay the same action sequence on the oracle
                 trace.append((action.clone(), None, None))
             if record is not None:
@@ -201,10 +217,11 @@ class _MatchBuffers:
     """Fixed-address inputs and outputs of brl_duplicate_match for one shape (n envs, M nets, P ranges; P = 0: one range
     over the batch), so that repeated calls relaunch the op's cached graph instead of capturing a new one."""
 
-    def __init__(self, n: int, M: int, P: int, dev, with_models: bool, with_tables: bool, pool=None):
+    def __init__(self, n: int, M: int, P: int, dev, with_models: bool, with_tables: bool, pool=None, players: bool = False):
         self.keys = torch.empty(n, dtype=torch.int64, device=dev)
         self.pool = pool if pool is not None else torch.zeros((M, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
-        self.env_models = torch.empty((n, 2), dtype=torch.int32, device=dev) if with_models else None
+        # a net per team, or with `players` per player id (BRL_F_PLAYER_MODELS)
+        self.env_models = torch.empty((n, 4 if players else 2), dtype=torch.int32, device=dev) if with_models else None
         self.offsets = torch.empty(P + 1, dtype=torch.int64, device=dev) if P else None
         self.scratch = torch.empty(ops.duplicate_match_scratch_bytes(n, M), dtype=torch.uint8, device=dev)
         self.cum_return = torch.empty(n, dtype=torch.float32, device=dev)
@@ -242,26 +259,37 @@ def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_en
     Same contract -- `duplicate_evaluate(team1_params, team2_params, rng_key) -> (log_info, table_a_info, table_b_info,
     cum_return)`, same key split and keys, one all-reduce of f64[8] over the ranks -- and the same per-env results.
     Both teams share `activation` / `model_type` (the pool holds one architecture).  `record` / `trace` need per-step host
-    copies: use make_simple_duplicate_evaluate for them.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path."""
+    copies: use make_simple_duplicate_evaluate for them.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path.
+    `team1_partner`: player 1's net instead of team1_params, which then plays player 0 only (a 3-net pool with nets by
+    player id, BRL_F_PLAYER_MODELS; its own buffers and graph)."""
     forward_pass = make_forward_pass(activation=activation, model_type=model_type)
     n, dev = num_eval_envs, eval_env.device
     bufs = _MatchBuffers(n, 2, 0, dev, with_models=False, with_tables=True)
+    partner_bufs = []                                           # allocated at the first call with a partner
     blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
 
-    def duplicate_evaluate(team1_params, team2_params, rng_key):
+    def duplicate_evaluate(team1_params, team2_params, rng_key, team1_partner=None):
+        if team1_partner is not None:
+            if not partner_bufs:
+                partner_bufs.append(_MatchBuffers(n, 3, 0, dev, with_models=True, with_tables=True, players=True))
+                partner_bufs[0].env_models.copy_(torch.tensor([0, 2, 1, 1], dtype=torch.int32, device=dev).expand(n, 4))
+            b = partner_bufs[0]
+            forward_pass.pack_into(team1_partner, b.pool[2, :blob_bytes])
+        else:
+            b = bufs
         rng_key, sub_key = brandom.split(rng_key)
-        bufs.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))                       # :93-94
-        forward_pass.pack_into(team1_params, bufs.pool[0, :blob_bytes])
-        forward_pass.pack_into(team2_params, bufs.pool[1, :blob_bytes])
-        bufs.play(eval_env, forward_pass.precision == "tc-bf16", tune)                      # :95-198
-        sums = bufs.sums.clone()
+        b.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))                          # :93-94
+        forward_pass.pack_into(team1_params, b.pool[0, :blob_bytes])
+        forward_pass.pack_into(team2_params, b.pool[1, :blob_bytes])
+        b.play(eval_env, forward_pass.precision == "tc-bf16", tune)                         # :95-198
+        sums = b.sums.clone()
         bdist.allreduce_sums(sums)
-        host = torch.cat((sums, bufs.status.to(torch.float64))).cpu()
+        host = torch.cat((sums, b.status.to(torch.float64))).cpu()
         _check_match_status(int(host[8]))
         log_info = bdist.stats_from_sums(host[:8])                                        # :199-201
         infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
-                            t.call_xx.clone()) for t in bufs.tables]
-        return log_info, infos[0], infos[1], bufs.cum_return.clone()
+                            t.call_xx.clone()) for t in b.tables]
+        return log_info, infos[0], infos[1], b.cum_return.clone()
 
     return duplicate_evaluate
 
@@ -301,10 +329,11 @@ def pfsp_probe_bytes(capacity: int, num_eval_envs: int, max_envs: int = 1 << 20,
 
 
 def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_envs: int, tune: int):
-    """The engine of the self-play league and the PFSP probe: `matches(pairs, rng_key, params_list=None, pool=None,
+    """The engine of the self-play league, the PFSP probe and cross-play: `matches(pairs, rng_key, params_list=None, pool=None,
     cum_returns=None)` plays every (i, j) of `pairs` -- net i of the pool on players 0/1, net j on 2/3 -- as the duplicate match
     `make_simple_duplicate_evaluate(..., num_eval_envs)(net_i, net_j, rng_key)` plays, on the same boards in every match, and
-    returns their (imp, se, win_rate) in `pairs` order.  The nets are `params_list` (packed into a pool of the matches' own)
+    returns their (imp, se, win_rate) in `pairs` order.  `pairs` may instead hold 4-tuples (a, b, c, d): net a on player 0,
+    b on 1, c on 2 and d on 3 (env_models[n, 4] by player id, BRL_F_PLAYER_MODELS; with `params_list` only).  The nets are `params_list` (packed into a pool of the matches' own)
     or the caller's packed `pool` (u8[M, brl_mlp_pool_stride()], used in place).  At most `max_envs` envs per rank make one
     chunk and one brl_duplicate_match call; a chunk's envs are sharded by global index over the ranks (pair_chunk_layout),
     with one all-reduce of f64[P, 8] and one host read per chunk, so the result does not depend on the rank count.
@@ -332,11 +361,14 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
 
     def matches(pairs, rng_key, params_list=None, pool=None, cum_returns=None):
         M = len(params_list) if pool is None else pool.shape[0]
+        width = len(pairs[0]) if len(pairs) else 2             # nets by team (i, j) or by player (a, b, c, d)
+        if width not in (2, 4) or any(len(p) != width for p in pairs) or (width == 4 and pool is not None):
+            raise ValueError("matches: pairs are all (i, j), or all (a, b, c, d) with params_list")
         if pool is not None:
             reserve(pool, len(pairs))
         _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
         board_keys = eval_env.make_keys(sub_key, n)
-        pair_arr = np.asarray(pairs, dtype=np.int32).reshape(-1, 2)
+        pair_arr = np.asarray(pairs, dtype=np.int32).reshape(-1, width)
         stats = []
         for c0, P, lo, hi, p_lo, p_hi, bounds in pair_chunk_layout(len(pairs), n, pairs_per_chunk, rank, world):
             sums = torch.zeros((P, 8), dtype=torch.float64, device=dev)
@@ -346,9 +378,10 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
                 if pool is not None:
                     b = held["buffers"].prefix(hi - lo, p_hi - p_lo)
                 else:
-                    key = (hi - lo, M, p_hi - p_lo)
+                    key = (hi - lo, M, p_hi - p_lo, width)
                     if key not in buffers:
-                        buffers[key] = _MatchBuffers(hi - lo, M, p_hi - p_lo, dev, with_models=True, with_tables=False)
+                        buffers[key] = _MatchBuffers(hi - lo, M, p_hi - p_lo, dev, with_models=True, with_tables=False,
+                                                     players=width == 4)
                     b = buffers[key]
                     for m, params in enumerate(params_list):
                         forward_pass.pack_into(params, b.pool[m, :blob_bytes])
@@ -394,6 +427,36 @@ def make_selfplay_league_evaluate(eval_env, activation, model_type, num_eval_env
         return (stats,) + league_matrices(M, {pair: s[0] for pair, s in stats.items()})
 
     return league
+
+
+def make_crossplay_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):
+    """Cross-play: how well the nets of a pool bid together as partners.  `crossplay(params_list, opponents, rng_key,
+    cum_returns=None)` plays every ordered partnership (a, b) of the M nets of `params_list` -- net a on player 0, net b on
+    player 1, the diagonal (a, a) included -- against the fixed pair `opponents` = (c, d) on players 2 / 3, each the duplicate
+    match `make_simple_duplicate_evaluate(..., num_eval_envs)(a, c, rng_key, team1_partner=b, team2_partner=d)` plays, on the
+    same boards in every match.  The M^2 matches are chunked and sharded as the self-play league's (at most `max_envs` envs
+    per rank a chunk, one brl_duplicate_match call each over a pool of the M + 2 nets with the nets by player id), so the
+    result does not depend on the rank count.  Returns ({(a, b): (imp, se, win_rate)}, imp[M, M]) with imp[a, b] the mean
+    IMP of partnership (a, b); (a, a) against (c, c) is `make_device_duplicate_evaluate(...)(a, c, rng_key)`'s.
+    `cum_returns` (a dict, tests) receives each partnership's per-env returns of this rank's shard under (a, b).  `tune`:
+    BRL_F_TUNE_MLP_* bits pinning the forward's path."""
+    import numpy as np
+    matches = _make_device_pair_matches(eval_env, make_forward_pass(activation=activation, model_type=model_type),
+                                        num_eval_envs, max_envs, tune)
+
+    def crossplay(params_list, opponents, rng_key, cum_returns=None):
+        M = len(params_list)
+        c, d = opponents
+        pairs = [(a, b, M, M + 1) for a in range(M) for b in range(M)]
+        by_pair = {} if cum_returns is not None else None
+        stats = dict(zip(((a, b) for a, b, _, _ in pairs),
+                         matches(pairs, rng_key, params_list=list(params_list) + [c, d], cum_returns=by_pair)))
+        if cum_returns is not None:
+            cum_returns.update({pair[:2]: v for pair, v in by_pair.items()})
+        imp = np.array([[stats[(a, b)][0] for b in range(M)] for a in range(M)], dtype=np.float64).reshape(M, M)
+        return stats, imp
+
+    return crossplay
 
 
 def make_device_pfsp_probe(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):
@@ -463,7 +526,8 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
     `team2_model_path`, or always-pass in "free-run"); every decision is the masked argmax.  Besides the score it
     logs, per team, the unmasked probability mass on illegal actions, bid / contract histograms and declarer /
     double / make / down / pass-out ratios.  `num_eval_envs` is this rank's shard; the statistics are all-reduced
-    (one collective) when torch.distributed is initialised."""
+    (one collective) when torch.distributed is initialised.  Both evaluators take `partner_params`: player 1's net (of the
+    actor's architecture) instead of the actor, which then plays player 0 only."""
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
     if game_mode == "competitive":
@@ -475,7 +539,7 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
     n, dev = num_eval_envs, eval_env.device
     n_sums = ops._lib.load().brl_eval_num_sums()
 
-    def _loop(actor_params, rng_key, step, state, trace):
+    def _loop(actor_params, rng_key, step, state, trace, partner_params):
         acc = torch.zeros((n, ops._lib.EVAL_ACC_COLS), dtype=torch.float32, device=dev)
         cum_return = torch.zeros(n, dtype=torch.float32, device=dev)
         rewards = torch.zeros((n, 4), dtype=torch.float32, device=dev)
@@ -487,7 +551,7 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
             rows1, rows2 = teams.split(state.current_player, state._terminated_u8)
             if rows1.shape[0] + rows2.shape[0] == 0:
                 return state, acc, cum_return, rewards
-            actor_forward_pass.act_rows(actor_params, state.observation, state._mask_u8, action, rows1, logits=logits)
+            _act_team(actor_forward_pass, actor_params, partner_params, state, action, rows1, logits=logits)
             if opp_params is not None:
                 opp_forward_pass.act_rows(opp_params, state.observation, state._mask_u8, action, rows2, logits=logits)
             # the step's decision + update_log_info (unmasked-softmax illegal mass, bid histograms) from the acting
@@ -501,11 +565,11 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
             rewards += state.rewards
             cum_return += state.rewards[:, 0]
 
-    def evaluate(actor_params, rng_key, trace=None):
+    def evaluate(actor_params, rng_key, trace=None, partner_params=None):
         rng_key, sub_key = brandom.split(rng_key)
         state = _bf16_state(eval_env, eval_env.make_keys(sub_key, n, env_offset))
         state, acc, cum_return, rewards = _loop(actor_params, rng_key, lambda s, a: eval_env.step(s, a, inplace=True),
-                                                state, trace)
+                                                state, trace, partner_params)
         f = ops.state_fields(state._packed)
         sums = torch.zeros(n_sums, dtype=torch.float64, device=dev)
         ops.eval_summary(acc, cum_return, f["step_count"],
@@ -514,7 +578,7 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
         state.rewards.copy_(rewards)                                                   # state.replace(rewards=rewards), :574
         return state, _log_info_from_sums(sums.cpu().numpy(), duplicate=False)
 
-    def duplicate_evaluate(actor_params, rng_key, trace=None):
+    def duplicate_evaluate(actor_params, rng_key, trace=None, partner_params=None):
         step_fn = duplicate_step(eval_env.step)
         rng_key, sub_key = brandom.split(rng_key)
         state = _bf16_state(eval_env, eval_env.make_keys(sub_key, n, env_offset))
@@ -524,7 +588,7 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
             s, infos[0], infos[1] = step_fn(s, a, infos[0], infos[1])
             return s
 
-        state, acc, cum_return, _ = _loop(actor_params, rng_key, step, state, trace)
+        state, acc, cum_return, _ = _loop(actor_params, rng_key, step, state, trace, partner_params)
         f = ops.state_fields(state._packed)
         sums = torch.zeros(n_sums, dtype=torch.float64, device=dev)
         tv = lambda t: (t.last_bid, t.last_bidder, t.call_x.view(torch.uint8), t.call_xx.view(torch.uint8), t.rewards, None)  # noqa: E731
@@ -565,12 +629,12 @@ class _EvalBuffers:
     """Fixed-address inputs and outputs of brl_evaluate_match for one shape and mode (as _MatchBuffers: repeated calls
     relaunch the op's cached graph)."""
 
-    def __init__(self, n: int, mode: int, dev):
+    def __init__(self, n: int, mode: int, dev, partner: bool = False):
         L = ops._lib
-        self.mode = mode
+        self.mode, self.partner = mode, partner
         self.keys = torch.empty(n, dtype=torch.int64, device=dev)
-        self.pool = torch.zeros((2, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
-        self.scratch = torch.empty(ops.evaluate_match_scratch_bytes(n, mode), dtype=torch.uint8, device=dev)
+        self.pool = torch.zeros((3 if partner else 2, ops.mlp_pool_stride()), dtype=torch.uint8, device=dev)
+        self.scratch = torch.empty(ops.evaluate_match_scratch_bytes(n, mode, partner), dtype=torch.uint8, device=dev)
         self.cum_return = torch.empty(n, dtype=torch.float32, device=dev)
         self.status = torch.zeros(1, dtype=torch.int32, device=dev)
         full = mode != L.EVAL_MATCH_SIMPLE
@@ -587,7 +651,8 @@ class _EvalBuffers:
             self.sums.zero_()
         ops.evaluate_match(self.keys, eval_env.table, self.pool, self.scratch, self.cum_return, self.status, mode=self.mode,
                            acc=self.acc, sums=self.sums, table_a=self.tables[0], table_b=self.tables[1],
-                           final_state=self.final_state, final=self.final, free_run=free_run, single_bf16=single_bf16, tune=tune,
+                           final_state=self.final_state, final=self.final, free_run=free_run, partner=self.partner,
+                           single_bf16=single_bf16, tune=tune,
                            illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
 
 
@@ -606,6 +671,7 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
     (state, log_info)`, same key split and keys, `env_offset` sharding, one all-reduce of the statistics over the ranks -- and
     the same per-env results.  In "free-run" team 2's rows are forwarded by the actor's net and not read (brl_evaluate_match).
     `trace` needs per-step host copies: use make_evaluate for it.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path.
+    `partner_params`: player 1's net instead of the actor (BRL_F_EVAL_PARTNER, its own buffers and graph).
     The returned function's `buffers` hold the last call's per-env `acc` rows and `cum_return`."""
     L = ops._lib
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
@@ -618,15 +684,22 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
         raise ValueError(game_mode)
     single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
     n, dev = num_eval_envs, eval_env.device
-    bufs = _EvalBuffers(n, L.EVAL_MATCH_DUPLICATE if duplicate else L.EVAL_MATCH_SINGLE, dev)
+    mode = L.EVAL_MATCH_DUPLICATE if duplicate else L.EVAL_MATCH_SINGLE
+    sets = {False: _EvalBuffers(n, mode, dev)}                  # with a partner: a 3-net set, allocated at its first call
     blob_bytes = L.load().brl_mlp_packed_bytes()
 
-    def play(actor_params, rng_key):
+    def play(actor_params, rng_key, partner_params):
+        partnered = partner_params is not None
+        if partnered not in sets:
+            sets[partnered] = _EvalBuffers(n, mode, dev, partner=True)
+        fn.buffers = bufs = sets[partnered]
         rng_key, sub_key = brandom.split(rng_key)
         bufs.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))
         actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
         if opp_params is not None:
             opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
+        if partnered:
+            actor_forward_pass.pack_into(partner_params, bufs.pool[2, :blob_bytes])
         bufs.play(eval_env, single_bf16, opp_params is None, tune)
         sums = bufs.sums.clone()
         bdist.allreduce_sums(sums)
@@ -634,22 +707,22 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
         _check_match_status(int(host[-1]), "brl_evaluate_match")
         return host[:-1]
 
-    def evaluate(actor_params, rng_key):
-        sums = play(actor_params, rng_key)
+    def evaluate(actor_params, rng_key, partner_params=None):
+        sums = play(actor_params, rng_key, partner_params)
         from .env import State
         out = ops.EnvOutputs(n, dev, torch.bfloat16)
         for k in ops.EnvOutputs.__slots__:
-            getattr(out, k).copy_(getattr(bufs.final, k))
-        return State(eval_env, bufs.final_state.clone(), out), _log_info_from_sums(sums, duplicate=False)
+            getattr(out, k).copy_(getattr(fn.buffers.final, k))
+        return State(eval_env, fn.buffers.final_state.clone(), out), _log_info_from_sums(sums, duplicate=False)
 
-    def duplicate_evaluate(actor_params, rng_key):
-        sums = play(actor_params, rng_key)
+    def duplicate_evaluate(actor_params, rng_key, partner_params=None):
+        sums = play(actor_params, rng_key, partner_params)
         infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
-                            t.call_xx.clone()) for t in bufs.tables]
+                            t.call_xx.clone()) for t in fn.buffers.tables]
         return _log_info_from_sums(sums, duplicate=True), infos[0], infos[1]
 
     fn = duplicate_evaluate if duplicate else evaluate
-    fn.buffers = bufs
+    fn.buffers = sets[False]
     return fn
 
 
@@ -676,23 +749,30 @@ def make_device_simple_evaluate(eval_env, team1_activation, team1_model_type, te
     `simple_evaluate(actor_params, rng) -> R.mean()`.  Every decision is an argmax and the net acting is fixed per seat, so the
     device loop takes one env step per iteration and forwards each live env through the one net that acts there, where the
     host loop forwards both nets over every env until the last auction ends.  `trace` needs per-step host copies: use
-    make_simple_evaluate for it.  The returned function's `buffers.cum_return` holds the last call's R."""
+    make_simple_evaluate for it.  `partner_params`: the net of the initial player's partner instead of the actor
+    (BRL_F_EVAL_PARTNER, its own buffers and graph).  The returned function's `buffers.cum_return` holds the last call's R."""
     L = ops._lib
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
     opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
     single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
-    bufs = _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device)
+    sets = {False: _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device)}
     blob_bytes = L.load().brl_mlp_packed_bytes()
 
-    def simple_evaluate(actor_params, rng):
+    def simple_evaluate(actor_params, rng, partner_params=None):
+        partnered = partner_params is not None
+        if partnered not in sets:
+            sets[partnered] = _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device, partner=True)
+        simple_evaluate.buffers = bufs = sets[partnered]
         rng_key, sub_key = brandom.split(rng)
         bufs.keys.copy_(eval_env.make_keys(sub_key, num_eval_envs))
         actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
         opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
+        if partnered:
+            actor_forward_pass.pack_into(partner_params, bufs.pool[2, :blob_bytes])
         bufs.play(eval_env, single_bf16, False, tune)
         _check_match_status(int(bufs.status[0]), "brl_evaluate_match")
         return bufs.cum_return.mean()
 
-    simple_evaluate.buffers = bufs
+    simple_evaluate.buffers = sets[False]
     return simple_evaluate

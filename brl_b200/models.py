@@ -47,6 +47,19 @@ def load_params(path: str, device="cuda") -> Dict[str, Dict[str, torch.Tensor]]:
             for k, v in raw.items()}
 
 
+def check_params_file(path: str) -> None:
+    """ValueError unless the pickle at `path` holds a DeepMind 4x1024 net (the LAYERS, each 'w' / 'b' of the SIZES), read on
+    the host only -- so a wrong file is refused before any device work"""
+    with open(path, "rb") as fh:
+        raw = _NoJaxUnpickler(io.BytesIO(fh.read())).load()
+    if not isinstance(raw, dict) or set(raw) != set(LAYERS):
+        raise ValueError(f"{path}: not a DeepMind 4x1024 parameter set (layers {sorted(raw) if isinstance(raw, dict) else type(raw)})")
+    for name, (fi, fo) in zip(LAYERS, SIZES):
+        shapes = {k: tuple(np.shape(raw[name].get(k))) for k in ("w", "b")} if isinstance(raw[name], dict) else {}
+        if shapes != {"w": (fi, fo), "b": (fo,)}:
+            raise ValueError(f"{path}: {name} has shapes {shapes}, not w {(fi, fo)} / b {(fo,)} of the DeepMind 4x1024 net")
+
+
 def init_params(seed: int, device="cuda") -> Dict[str, Dict[str, torch.Tensor]]:
     """Random-init weights of the architecture: haiku's default `hk.initializers.TruncatedNormal(stddev=1/sqrt(fan_in))`,
     i.e. a standard normal truncated to [-2, 2] by RESAMPLING (not clipping), scaled by 1/sqrt(fan_in); biases zero."""

@@ -675,17 +675,19 @@ def mlp_pack_pool(params_list, pack_one) -> torch.Tensor:
 
 def model_rows(current_player: torch.Tensor, done: Optional[torch.Tensor], env_models: torch.Tensor, rows: torch.Tensor,
                counts: torch.Tensor, offsets: torch.Tensor, block_model: torch.Tensor) -> None:
-    """Live envs (done == 0) grouped by the net that acts there: env_models[i, 0] for players 0/1, [i, 1] for players 2/3.
-    Net m's rows are rows[offsets[m] : offsets[m] + counts[m]], padded with -1 to offsets[m + 1]; offsets[M] is the padded
+    """Live envs (done == 0) grouped by the net that acts there: env_models[i, 0] for players 0/1, [i, 1] for players 2/3,
+    or, with env_models int32[n, 4], env_models[i, player] for each player id (BRL_F_PLAYER_MODELS).  Net m's rows are rows[offsets[m] : offsets[m] + counts[m]], padded with -1 to offsets[m + 1]; offsets[M] is the padded
     row count and block_model the net of each 256-row block.  A live env whose id is outside [0, M) makes offsets[M] = -1:
     the grouping is invalid, and the caller's read of offsets[M] (which sizes the forward) must raise."""
     n_models = counts.shape[0]
-    if env_models.dtype != torch.int32 or tuple(env_models.shape) != (current_player.shape[0], 2):
-        raise _lib.BrlError("model_rows: env_models must be int32 [n, 2]")
+    if env_models.dtype != torch.int32 or env_models.dim() != 2 or tuple(env_models.shape) not in \
+            ((current_player.shape[0], 2), (current_player.shape[0], 4)):
+        raise _lib.BrlError("model_rows: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
     if offsets.shape[0] != n_models + 1 or rows.shape[0] < model_rows_capacity(current_player.shape[0], n_models):
         raise _lib.BrlError("model_rows: offsets must hold M + 1 entries and rows model_rows_capacity(n, M)")
+    flags = _lib.F_PLAYER_MODELS if env_models.shape[1] == 4 else 0
     _call("brl_model_rows", [_ptr(current_player), _ptr(done), _ptr(env_models), _ptr(rows), _ptr(counts), _ptr(offsets),
-                             _ptr(block_model)], _params(current_player.shape[0], k_steps=n_models))
+                             _ptr(block_model)], _params(current_player.shape[0], k_steps=n_models, flags=flags))
 
 
 def policy_act_grouped(obs_bf16: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, mask: Optional[torch.Tensor],
@@ -742,14 +744,16 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
                     illegal_penalty: float = -1.0, illegal_bonus: float = 1.0) -> None:
     """Play duplicate_evaluate's whole loop (src/evaluation.py:93-201) for every env of `keys` in one call, with the loop on
     the device: env e plays net env_models[e, 0] of `pool` on players 0/1 against env_models[e, 1] on 2/3 (default: net 0
-    against net 1, M must be 2).  Writes cum_return f32[n], adds the match sums to `sums` (f64[P, 8] over the ranges of
+    against net 1, M must be 2), or with env_models int32[n, 4] net env_models[e, p] on player p (BRL_F_PLAYER_MODELS: each
+    partner may be a different net).  Writes cum_return f32[n], adds the match sums to `sums` (f64[P, 8] over the ranges of
     `range_offsets` int64[P + 1], or f64[8] for the whole batch), the status (int32[1], _lib.MATCH_*) and, when given, the
     final Table_info of both tables.  Nothing is read back to the host; read `status` with the sums."""
     n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
     if env_models is None and M != 2:
         raise _lib.BrlError(f"duplicate_match: without env_models the pool must hold 2 nets, got {M}")
-    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) != (n, 2)):
-        raise _lib.BrlError("duplicate_match: env_models must be int32 [n, 2]")
+    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4))):
+        raise _lib.BrlError("duplicate_match: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    player_models = env_models is not None and env_models.shape[1] == 4
     P = 0
     if range_offsets is not None:
         P = int(range_offsets.shape[0]) - 1
@@ -768,20 +772,24 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
     infos = table_a.ptrs() + table_b.ptrs() if table_a is not None else [None] * 12
     _call("brl_duplicate_match", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(env_models), _ptr(range_offsets), _ptr(scratch),
                                   _ptr(cum_return), _ptr(sums), _ptr(status)] + infos,
-          _params(n, k_steps=M, step=P, n_deals=table.shape[0], flags=(F_MLP_BF16 if single_bf16 else 0) | tune,
+          _params(n, k_steps=M, step=P, n_deals=table.shape[0],
+                  flags=(F_MLP_BF16 if single_bf16 else 0) | (_lib.F_PLAYER_MODELS if player_models else 0) | tune,
                   illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))
 
 
 # ---- a whole evaluation as one call (ppo.py:365-374; src/evaluation.py:11-66, 207-1032) -----------------------------------
-def evaluate_match_scratch_bytes(n_envs: int, mode: int) -> int:
-    return _size_query("brl_evaluate_match_scratch_bytes", n_envs, mode)
+def evaluate_match_scratch_bytes(n_envs: int, mode: int, partner: bool = False) -> int:
+    """scratch bytes of `evaluate_match` for n_envs envs in `mode`, with or without the partner's net in the pool"""
+    name = "brl_evaluate_match_partner_scratch_bytes" if partner else "brl_evaluate_match_scratch_bytes"
+    return _size_query(name, n_envs, mode)
 
 
 def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, scratch: torch.Tensor, cum_return: torch.Tensor,
                    status: torch.Tensor, *, mode: int, acc: Optional[torch.Tensor] = None, sums: Optional[torch.Tensor] = None,
                    table_a: Optional[TableInfoBuffers] = None, table_b: Optional[TableInfoBuffers] = None,
                    final_state: Optional[torch.Tensor] = None, final: Optional[EnvOutputs] = None, free_run: bool = False,
-                   single_bf16: bool = False, tune: int = 0, illegal_penalty: float = -1.0, illegal_bonus: float = 1.0) -> None:
+                   partner: bool = False, single_bf16: bool = False, tune: int = 0, illegal_penalty: float = -1.0,
+                   illegal_bonus: float = 1.0) -> None:
     """Play a whole evaluation (make_evaluate's duplicate_evaluate / evaluate, or make_simple_evaluate) for every env of `keys`
     in one call, with the loop on the device.  `pool` u8[2, mlp_pool_stride()]: net 0 is team 1 / the actor, net 1 team 2 / the
     opponent (not read with free_run).  `mode` = _lib.EVAL_MATCH_*:
@@ -789,6 +797,9 @@ def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, 
         (f64[brl_eval_num_sums()]); DUPLICATE writes the final Table_infos when given, SINGLE the final state (`final_state`
         int32[5, n, 4], `final` with a bf16 observation; its rewards = the summed step rewards) when given;
       SIMPLE: cum_return = R, the per-env return of the player to act at the start.
+    `partner` (BRL_F_EVAL_PARTNER): `pool` is u8[3, mlp_pool_stride()] and net 2 plays the actor's partner -- player 1 in
+    DUPLICATE / SINGLE, the initial player's partner in SIMPLE -- with the scratch of evaluate_match_scratch_bytes(n, mode,
+    partner=True).
     `status` (int32[1], _lib.MATCH_*) is written too; nothing is read back to the host."""
     n = int(keys.shape[0])
     if mode not in (_lib.EVAL_MATCH_DUPLICATE, _lib.EVAL_MATCH_SINGLE, _lib.EVAL_MATCH_SIMPLE):
@@ -796,15 +807,17 @@ def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, 
     full = mode != _lib.EVAL_MATCH_SIMPLE
     if free_run and not full:
         raise _lib.BrlError("evaluate_match: free_run is a mode of the full-statistics evaluation")
-    if pool.dim() != 2 or pool.dtype != torch.uint8 or tuple(pool.shape) != (2, mlp_pool_stride()):
-        raise _lib.BrlError("evaluate_match: pool must be u8[2, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    n_nets = 3 if partner else 2
+    if pool.dim() != 2 or pool.dtype != torch.uint8 or tuple(pool.shape) != (n_nets, mlp_pool_stride()):
+        raise _lib.BrlError(f"evaluate_match: pool must be u8[{n_nets}, mlp_pool_stride()] (ops.mlp_pack_pool)"
+                            + (" with the partner's net" if partner else ""))
     if cum_return.dtype != torch.float32 or status.dtype != torch.int32:
         raise _lib.BrlError("evaluate_match: cum_return must be float32 and status int32")
     if full:
         if acc is None or sums is None or acc.dtype != torch.float32 or tuple(acc.shape) != (n, _lib.EVAL_ACC_COLS) or \
                 sums.dtype != torch.float64 or sums.numel() != _lib.load().brl_eval_num_sums():
             raise _lib.BrlError("evaluate_match: full statistics need acc float32[n, 76] and sums float64[239]")
-    if scratch.numel() < evaluate_match_scratch_bytes(n, mode):
+    if scratch.numel() < evaluate_match_scratch_bytes(n, mode, partner):
         raise _lib.BrlError("evaluate_match: scratch too small (ops.evaluate_match_scratch_bytes)")
     if (table_a is None) != (table_b is None):
         raise _lib.BrlError("evaluate_match: give both Table_info outputs or neither")
@@ -815,6 +828,9 @@ def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, 
     infos = table_a.ptrs() + table_b.ptrs() if table_a is not None else [None] * 12
     finals = [_ptr(final_state)] + final.ptrs() if final is not None else [None] * 6
     flags = _lib.f_eval_match(mode) | (_lib.F_EVAL_FREE_RUN if free_run else 0) | (F_MLP_BF16 if single_bf16 else 0) | tune
+    if partner:
+        flags |= _lib.F_EVAL_PARTNER
     _call("brl_evaluate_match", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(scratch), _ptr(cum_return), _ptr(acc), _ptr(sums),
                                  _ptr(status)] + infos + finals,
-          _params(n, n_deals=table.shape[0], flags=flags, illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))
+          _params(n, n_deals=table.shape[0], flags=flags, k_steps=3 if partner else 0, illegal_penalty=illegal_penalty,
+                  illegal_bonus=illegal_bonus))

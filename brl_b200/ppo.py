@@ -12,6 +12,11 @@ score / reward_scale (roll_out.py), and `log_par=True` adds eval/imp_vs_par, eva
 of the eval/* duplicate match to the iterations that play it (evaluation.par_statistics).  The defaults ("score", False)
 leave every code path as it was.
 
+Fixed partner (not in the reference; DESIGN.md f14): `partner_model_path` names a DeepMind 4x1024 net that bids as the
+learner's partner.  It plays the roll-out's sub-step 3 (the partner slot of the quad step) and is team 1's partner in
+train/score, the imp_opp_before / imp_opp_after probes and the eval/* match (log_par's too); the opponent team stays
+(opp, opp) and the partner is not trained.  Unset (the default), every code path is the one without the feature.
+
 Everything heavy runs in the kernels behind `brl_b200.ops`; this file is the control
 plane only (config defaults, opponent selection, table rotation, logging hooks).  wandb,
 OmegaConf and the dataset download are out of scope (SURVEY 2): `log_fn` receives the same
@@ -37,7 +42,7 @@ from .env import BridgeBidding
 from .evaluation import (make_device_duplicate_evaluate, make_device_evaluate, make_device_pfsp_probe,
                          make_device_simple_evaluate, make_evaluate_log, par_statistics)
 from .gae import make_calc_gae
-from .models import LAYERS, ForwardPass, init_params, load_params, make_forward_pass
+from .models import LAYERS, ForwardPass, check_params_file, init_params, load_params, make_forward_pass
 from .optim import OptState, make_optimizer
 from .pbt import default_pbt_config  # noqa: F401 -- ppo.default_pbt_config(): the options of train_population's `pbt`
 from .roll_out import check_reward_mode, make_roll_out
@@ -60,7 +65,7 @@ def default_config() -> dict:
         value_clipping=True, global_gradient_clipping=True, anneal_lr=False, reward_scaling=False, max_grad_norm=0.5,
         reward_scale=7600.0, actor_illegal_action_mask=True, actor_illegal_action_penalty=False,
         illegal_action_penalty=-1.0, illegal_action_l2norm_coef=0.0, anchor_model_path=None, anchor_kl_coef=0.0,
-        reward_mode="score", log_par=False)
+        reward_mode="score", log_par=False, partner_model_path=None)
 
 
 def check_anchor_config(config: dict) -> None:
@@ -70,6 +75,18 @@ def check_anchor_config(config: dict) -> None:
         raise ValueError(f"anchor_kl_coef must be a finite number >= 0; got {coef!r}")
     if coef != 0 and not config.get("anchor_model_path"):
         raise ValueError(f"anchor_kl_coef = {coef!r} needs an anchor net: set anchor_model_path")
+
+
+def check_partner_config(config: dict) -> None:
+    """ValueError for a partner_model_path together with ratio_model_zoo > 0 (zoo opponents have no partner slot), and for a
+    file that is not a DeepMind 4x1024 parameter set; reads the file on the host only"""
+    path = config.get("partner_model_path")
+    if not path:
+        return
+    if float(config.get("ratio_model_zoo", 0.0)) > 0.0:
+        raise ValueError("partner_model_path cannot be combined with ratio_model_zoo > 0: FSP / PFSP zoo opponents are "
+                         "played without a partner")
+    check_params_file(path)
 
 
 def params_to_host(params) -> dict:
@@ -123,6 +140,7 @@ class Learner:
         self.config = config = full_config(config)
         check_anchor_config(config)
         check_reward_mode(config)
+        check_partner_config(config)
         self.log_fn = log_fn
         self.np_rng = np_rng or np.random.default_rng(config["seed"])
         self.dev = dev = torch.device(device)
@@ -164,9 +182,14 @@ class Learner:
             self.anchor_params = load_params(config["anchor_model_path"], dev)
             anchor_forward_pass = make_fp(config["actor_activation"], config["actor_model_type"])
         self.anchor_logits = None  # the latest roll-out's anchor logits [num_steps, num_envs, 38]
+        # the fixed partner: a net of the actor's architecture, this learner's own (PBT's adopt keeps it), never trained
+        self.partner_params, partner_forward_pass = None, None
+        if config["partner_model_path"]:
+            self.partner_params = load_params(config["partner_model_path"], dev)
+            partner_forward_pass = make_fp(config["actor_activation"], config["actor_model_type"])
         self.envs = [BridgeBidding(table=t, device=dev) for t in tables]                              # ppo.py:296-303
-        self.roll_outs = [make_roll_out(config, env, self.actor_forward_pass, opp_forward_pass, anchor_forward_pass)
-                          for env in self.envs]
+        self.roll_outs = [make_roll_out(config, env, self.actor_forward_pass, opp_forward_pass, anchor_forward_pass,
+                                        partner_forward_pass) for env in self.envs]
         self.calc_gae = make_calc_gae(config, self.actor_forward_pass)
 
         rng, _rng = brandom.split(rng)
@@ -225,10 +248,11 @@ class Learner:
             if config["save_model"]:
                 save_params(runner_state[0], os.path.join(self.save_dir, f"params-{i:08}.pkl"))
         t0 = time.time()
-        self.R = self.simple_evaluate(runner_state[0], eval_rng)                                  # ppo.py:365-368
+        partner = self.partner_params
+        self.R = self.simple_evaluate(runner_state[0], eval_rng, partner_params=partner)          # ppo.py:365-368
         self.eval_log = {}
         if i % config["num_eval_step"] == 0:                                                      # ppo.py:369-374
-            log_info, table_a_info, table_b_info = self.duplicate_evaluate(runner_state[0], eval_rng)
+            log_info, table_a_info, table_b_info = self.duplicate_evaluate(runner_state[0], eval_rng, partner_params=partner)
             self.eval_log = make_evaluate_log(log_info)
             if config["log_par"]:  # the same match against par: its initial state from the keys it was played from
                 init_state = self.eval_env.init(self.duplicate_evaluate.buffers.keys)
@@ -239,7 +263,8 @@ class Learner:
         self.t_eval = time.time() - t0
 
         if config["self_play"]:                                                                   # ppo.py:376-470
-            (imp_opp, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng)
+            (imp_opp, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng,
+                                                                      team1_partner=partner)
             if imp_opp >= config["threshold_model_zoo"]:
                 if len(zoo) != 0 and np_rng.binomial(1, config["ratio_model_zoo"]):
                     if config["prioritized_fictitious"]:
@@ -256,10 +281,12 @@ class Learner:
                         self.opp_params = self.zoo_model(int(np_rng.integers(len(zoo))))
                 else:
                     self.opp_params = runner_state[0]
-        (self.imp_opp_before, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng)
+        (self.imp_opp_before, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, eval_rng,
+                                                                              team1_partner=partner)
         torch.cuda.synchronize(dev)
         t1 = time.time()
-        runner_state, traj_batch = self.roll_out(runner_state, self.opp_params, anchor_params=self.anchor_params)  # :472-475
+        runner_state, traj_batch = self.roll_out(runner_state, self.opp_params, anchor_params=self.anchor_params,
+                                                 partner_params=partner)                         # :472-475
         self.anchor_logits = self.roll_out.anchor_logits
         torch.cuda.synchronize(dev)
         t2 = time.time()
@@ -280,7 +307,8 @@ class Learner:
         per-minibatch KL to the anchor, [update_epochs, num_minibatches], logged as train/anchor_kl when there is an anchor."""
         config, dev = self.config, self.dev
         self.runner_state = runner_state
-        (imp_opp_after, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, self.eval_rng)
+        (imp_opp_after, _, _), _, _, _ = self.simple_duplicate_evaluate(runner_state[0], self.opp_params, self.eval_rng,
+                                                                        team1_partner=self.partner_params)
         self.steps += config["num_envs"] * config["num_steps"]
         total_loss, (value_loss, loss_actor, entropy, approx_kl, clipflacs, illegal_action_loss) = loss_info
         lr_now = self.optimizer.lr_at((i + 1) * config["update_epochs"] * config["num_minibatches"])
@@ -322,7 +350,7 @@ class Learner:
         """PBT's exploit and explore: take `src`'s parameters and Adam state (device copies into this learner's own
         buffers, on the current stream) and set the config `values`, rebuilding the optimizer that captured them.  The
         update step holds the loss coefficients and optimizers and is the caller's to rebuild.  Env state, rollout key,
-        table rotation, zoo, KL anchor and save directory stay this learner's; a self-play opponent becomes the new
+        table rotation, zoo, KL anchor, fixed partner and save directory stay this learner's; a self-play opponent becomes the new
         parameters."""
         params, opt_state = self.runner_state[:2]
         src_params, src_state = src.runner_state[:2]
@@ -391,7 +419,10 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
     None (the default) trains the learners independently, as above.
 
     KL anchors: each learner has its own anchor net (anchor_model_path) and coefficient (anchor_kl_coef, which PBT may
-    perturb); either every learner has an anchor or none has (ValueError naming anchor_model_path)."""
+    perturb); either every learner has an anchor or none has (ValueError naming anchor_model_path).
+
+    Fixed partners: each learner has its own partner_model_path or none (the partner is not trained, so the grouped update
+    is the same); every learner's partner is checked before any device work."""
     K = len(configs)
     if len(rngs) != K:
         raise ValueError("train_population needs one rng per config")
@@ -400,6 +431,7 @@ def train_population(configs: Sequence[dict], rngs: Sequence[int], tables: Optio
     for c in full:
         check_anchor_config(c)
         check_reward_mode(c)
+        check_partner_config(c)
     anchored = [bool(c["anchor_model_path"]) for c in full]
     if any(anchored) and not all(anchored):
         raise ValueError(f"population learners must all have a KL anchor or none: anchor_model_path is set for learners "

@@ -21,6 +21,11 @@ the anchor net on every step's observation (one `brl_mlp_forward` on the same bf
 trajectory, stays valid until the next call.  Anchored and plain calls keep separate buffers and CUDA graphs; the anchor
 is packed into its own fixed-address blob before an anchored replay.
 
+Partner (ppo.py `partner_model_path`): `roll_out(runner_state, opp_params, partner_params=...)` plays the quad step's
+sub-step 3 -- the actor's partner slot -- with that net instead of the actor (utils._QuadStep; sampled, not recorded).  That
+forward runs anyway, so a partner costs one more blob pack per graph replay: partnered calls keep their own buffers and
+CUDA graph, with the partner packed into its own fixed-address blob.
+
 Reward (config["reward_mode"]): "score" (the default) is the reference's rewards[actor] / reward_scale.  "par_imp" takes a
 finished board's reward against its double-dummy par (DESIGN.md f13) instead: IMP(rewards[actor] - par[actor]) / 24.  Before
 each quad step `brl_par` writes the par of the state in `buf.packed` into the rollout's `par[n, 4]`: that state still holds
@@ -112,7 +117,7 @@ class _Buffers:
             self.player[0].copy_(env_state.current_player)
 
 
-def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forward_pass=None):
+def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forward_pass=None, partner_forward_pass=None):
     masked = bool(config["actor_illegal_action_mask"])
     if not masked and not config.get("actor_illegal_action_penalty", False):
         raise ValueError("one of actor_illegal_action_mask / actor_illegal_action_penalty must be set (src/roll_out.py:24-39)")
@@ -128,13 +133,15 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
     T = int(config["num_steps"])
     scale = float(config["reward_scale"])
     obs_dtype = getattr(actor_forward_pass, "input_dtype", torch.float32)
-    cache = {}  # (n, anchored, reward_mode) -> dict(buf, graph, blobs, salt, anchor_logits, ...)
+    cache = {}  # (n, anchored, reward_mode, partnered) -> dict(buf, graph, blobs, salt, anchor_logits, ...)
     out = {"anchor_logits": None}
 
-    def body(buf, params, opp_params, rng, trace, anchor=None):
+    def body(buf, params, opp_params, rng, trace, anchor=None, partner_params=None):
         """the T steps of src/roll_out.py:49-108 on `buf`"""
         step_fn = make_step_fn(step_fn=auto_reset(env.step, env.init), actor_forward_pass=actor_forward_pass,
-                               actor_params=params, opp_forward_pass=opp_forward_pass, opp_params=opp_params)
+                               actor_params=params, opp_forward_pass=opp_forward_pass, opp_params=opp_params,
+                               partner_forward_pass=partner_forward_pass if partner_params is not None else None,
+                               partner_params=partner_params)
         step_fn.trace = trace
         cur = buf.state(env, 0)
         for t in range(T):
@@ -162,9 +169,10 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
                           log_prob=buf.log_prob, obs=buf.obs[:T], legal_action_mask=buf.mask[:T].view(torch.bool))
         return (params, opt_state, cur, cur.observation, total, rng), traj
 
-    def roll_out(runner_state, opp_params, anchor_params=None, trace=None, graph_seeding=False):
+    def roll_out(runner_state, opp_params, anchor_params=None, partner_params=None, trace=None, graph_seeding=False):
         """`anchor_params`: also record the anchor net's logits of every step in `roll_out.anchor_logits` (needs
-        `anchor_forward_pass`).  `trace` (tests): a list that receives every sub-step action tensor; forces the plain
+        `anchor_forward_pass`).  `partner_params`: the net of the quad step's sub-step 3 instead of the actor (needs
+        `partner_forward_pass`).  `trace` (tests): a list that receives every sub-step action tensor; forces the plain
         launch path.  `graph_seeding` (tests): plain launches with exactly the seeds a graph replay uses (captured constants
         XOR the per-rollout salt), so that a graph replay can be compared bit for bit with a traced, oracle-checked run."""
         params, opt_state, env_state, last_obs, terminated_count, rng = runner_state
@@ -172,13 +180,19 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
         anchored = anchor_params is not None
         if anchored and anchor_forward_pass is None:
             raise ValueError("roll_out got anchor_params, but make_roll_out was given no anchor_forward_pass")
+        partnered = partner_params is not None
+        if partnered and partner_forward_pass is None:
+            raise ValueError("roll_out got partner_params, but make_roll_out was given no partner_forward_pass")
         use_graph = trace is None and not graph_seeding and n >= _GRAPH_MIN_ENVS and \
             os.environ.get("BRL_ROLLOUT_GRAPH", "1") != "0" and \
             hasattr(actor_forward_pass, "pack_into") and hasattr(opp_forward_pass, "pack_into") and \
-            (not anchored or hasattr(anchor_forward_pass, "pack_into"))  # tensor-core nets only
-        c = cache.get((n, anchored, reward_mode))
+            (not anchored or hasattr(anchor_forward_pass, "pack_into")) and \
+            (not partnered or hasattr(partner_forward_pass, "pack_into"))  # tensor-core nets only
+        # the forward passes whose sampling seeds take the per-rollout salt
+        salted = (actor_forward_pass, opp_forward_pass) + ((partner_forward_pass,) if partnered else ())
+        c = cache.get((n, anchored, reward_mode, partnered))
         if c is None:
-            c = cache[(n, anchored, reward_mode)] = {"buf": _Buffers(T, n, dev, obs_dtype, par_mode), "graph": None}
+            c = cache[(n, anchored, reward_mode, partnered)] = {"buf": _Buffers(T, n, dev, obs_dtype, par_mode), "graph": None}
             if anchored:
                 c["anchor_logits"] = torch.empty((T, n, ops.NUM_ACTIONS), dtype=torch.float32, device=dev)
                 c["anchor_value"] = torch.empty(n, dtype=torch.float32, device=dev)
@@ -187,18 +201,20 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
         buf.load(env_state, last_obs)
         buf.count.zero_()
         if not use_graph:
-            prev = (getattr(actor_forward_pass, "seed_salt", None), getattr(opp_forward_pass, "seed_salt", None))
+            prev = [getattr(fp, "seed_salt", None) for fp in salted]
             salt, body_rng = None, rng
             if graph_seeding:
                 rng, key = brandom.split(rng)
                 salt = torch.tensor([key - (1 << 64) if key >= (1 << 63) else key], dtype=torch.int64, device=dev)
                 body_rng = _CAPTURE_KEY
-            actor_forward_pass.seed_salt = opp_forward_pass.seed_salt = salt
+            for fp in salted:
+                fp.seed_salt = salt
             anchor = (anchor_params, c["anchor_logits"], c["anchor_value"]) if anchored else None
             try:
-                cur, body_rng = body(buf, params, opp_params, body_rng, trace, anchor)
+                cur, body_rng = body(buf, params, opp_params, body_rng, trace, anchor, partner_params)
             finally:
-                actor_forward_pass.seed_salt, opp_forward_pass.seed_salt = prev
+                for fp, v in zip(reversed(salted), reversed(prev)):  # restored in reverse: a pass listed twice ends as it was
+                    fp.seed_salt = v
             return finish(buf, params, opt_state, cur, terminated_count, rng if graph_seeding else body_rng)
         # ---- CUDA-graph path ----
         if c["graph"] is None:
@@ -218,23 +234,31 @@ def make_roll_out(config, env, actor_forward_pass, opp_forward_pass, anchor_forw
                 c["anchor_blob"] = torch.empty(ops._lib.load().brl_mlp_packed_bytes(), dtype=torch.uint8, device=dev)
             anchor_forward_pass.pack_into(anchor_params, c["anchor_blob"])
             anchor = ({"_brl_packed_fixed": c["anchor_blob"]}, c["anchor_logits"], c["anchor_value"])
+        partner = None
+        if partnered:
+            if "partner_blob" not in c:
+                c["partner_blob"] = torch.empty(ops._lib.load().brl_mlp_packed_bytes(), dtype=torch.uint8, device=dev)
+            partner_forward_pass.pack_into(partner_params, c["partner_blob"])
+            partner = {"_brl_packed_fixed": c["partner_blob"]}
         if c["graph"] is None:
-            prev = (getattr(actor_forward_pass, "seed_salt", None), getattr(opp_forward_pass, "seed_salt", None))
-            actor_forward_pass.seed_salt = opp_forward_pass.seed_salt = c["salt"]  # baked into the captured launches only
+            prev = [getattr(fp, "seed_salt", None) for fp in salted]
+            for fp in salted:
+                fp.seed_salt = c["salt"]  # baked into the captured launches only
             saved = (buf.packed.clone(), buf.obs[0].clone(), buf.mask[0].clone(), buf.player[0].clone())
             side = torch.cuda.Stream(device=dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             try:
                 with torch.cuda.stream(side):
-                    body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor)  # warm-up: lazy allocations (scratch), attribute calls
+                    body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor, partner)  # warm-up: lazy allocations (scratch), attribute calls
                     buf.packed.copy_(saved[0]); buf.obs[0].copy_(saved[1]); buf.mask[0].copy_(saved[2]); buf.player[0].copy_(saved[3])
                     buf.count.zero_()
                     side.synchronize()
                     g = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g, stream=side):
-                        body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor)
+                        body(buf, fixed_a, fixed_o, _CAPTURE_KEY, None, anchor, partner)
             finally:
-                actor_forward_pass.seed_salt, opp_forward_pass.seed_salt = prev
+                for fp, v in zip(reversed(salted), reversed(prev)):
+                    fp.seed_salt = v
             torch.cuda.current_stream(dev).wait_stream(side)
             c["graph"] = g
             buf.packed.copy_(saved[0]); buf.obs[0].copy_(saved[1]); buf.mask[0].copy_(saved[2]); buf.player[0].copy_(saved[3])

@@ -63,12 +63,22 @@ def _env_of(step_fn):
 class _QuadStep:
     """Four consecutive env sub-steps (src/utils.py:69-128): the given action, then opp /
     actor / opp nets act on the fresh observation; returns the last state with
-    rewards = sum of the four and terminated = OR of the four."""
+    rewards = sum of the four and terminated = OR of the four.
 
-    def __init__(self, step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, mode: str):
+    Sub-step 3 is the partner's slot.  Given `partner_forward_pass` / `partner_params`, that net acts there instead of the
+    actor (still sampled in "sample" mode, and still no recorded transition).  The slot is positional, as in the reference:
+    after an auto-reset inside the quad step the seat to act at sub-step 3 may belong to the other team, and the partner's
+    net then acts for that team, as the actor's would without a partner."""
+
+    def __init__(self, step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, mode: str,
+                 partner_forward_pass=None, partner_params=None):
         self.env, self.autoreset = _env_of(step_fn)
         self.actor_fp, self.actor_params = actor_forward_pass, actor_params
         self.opp_fp, self.opp_params = opp_forward_pass, opp_params
+        if (partner_forward_pass is None) != (partner_params is None):
+            raise ValueError("a partner needs both partner_forward_pass and partner_params")
+        self.partner_fp, self.partner_params = (partner_forward_pass, partner_params) if partner_params is not None else \
+            (actor_forward_pass, actor_params)
         self.mode = mode  # "sample" | "deterministic" | "free-run"
         self._scratch = None
         self._mid_obs = None
@@ -94,7 +104,8 @@ class _QuadStep:
         # take bf16 input, write those straight in bf16 into a private buffer (no cast launch, half the bytes)
         mid = out
         if self.mode != "free-run" and getattr(self.actor_fp, "input_dtype", None) == torch.bfloat16 and \
-                getattr(self.opp_fp, "input_dtype", None) == torch.bfloat16 and out.observation.dtype != torch.bfloat16:
+                getattr(self.opp_fp, "input_dtype", None) == torch.bfloat16 and \
+                getattr(self.partner_fp, "input_dtype", None) == torch.bfloat16 and out.observation.dtype != torch.bfloat16:
             if self._mid_obs is None or self._mid_obs.shape[0] != n:
                 self._mid_obs = torch.empty((n, ops.OBS_DIM), dtype=torch.bfloat16, device=env.device)
             mid = State(env, packed, out).outputs()
@@ -103,7 +114,7 @@ class _QuadStep:
         if self.trace is not None:
             self.trace.append(action.clone())
         cur = State(env, packed, mid)
-        plan = ((self.opp_fp, self.opp_params), (self.actor_fp, self.actor_params), (self.opp_fp, self.opp_params))
+        plan = ((self.opp_fp, self.opp_params), (self.partner_fp, self.partner_params), (self.opp_fp, self.opp_params))
         for k, (fp, params) in enumerate(plan):
             rng, sub = brandom.split(rng)
             if self.mode == "free-run" and k != 1:
@@ -117,20 +128,26 @@ class _QuadStep:
         return State(env, packed, out)
 
 
-def single_play_step_two_policy_commpetitive(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params):
-    """src/utils.py:61-130 (sampled opponents / partner)"""
-    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "sample")
+def single_play_step_two_policy_commpetitive(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params,
+                                             partner_forward_pass=None, partner_params=None):
+    """src/utils.py:61-130 (sampled opponents / partner); the partner is the actor unless given"""
+    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "sample",
+                     partner_forward_pass, partner_params)
 
 
 def single_play_step_two_policy_commpetitive_deterministic(step_fn, actor_forward_pass, actor_params,
-                                                           opp_forward_pass, opp_params):
-    """src/utils.py:133-202 (argmax opponents / partner)"""
-    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "deterministic")
+                                                           opp_forward_pass, opp_params, partner_forward_pass=None,
+                                                           partner_params=None):
+    """src/utils.py:133-202 (argmax opponents / partner); the partner is the actor unless given"""
+    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "deterministic",
+                     partner_forward_pass, partner_params)
 
 
-def single_play_step_free_run(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params):
-    """src/utils.py:205-246 (opponents always pass, partner argmax)"""
-    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "free-run")
+def single_play_step_free_run(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params,
+                              partner_forward_pass=None, partner_params=None):
+    """src/utils.py:205-246 (opponents always pass, partner argmax); the partner is the actor unless given"""
+    return _QuadStep(step_fn, actor_forward_pass, actor_params, opp_forward_pass, opp_params, "free-run",
+                     partner_forward_pass, partner_params)
 
 
 def normal_step(step_fn):

@@ -314,7 +314,10 @@ int64_t brl_model_rows_capacity(int64_t n_envs, int64_t n_models);
  *          [3] out i32 rows[brl_model_rows_capacity(n, M)]: net m's live envs at [offsets[m], offsets[m] + counts[m]), then -1
  *              up to offsets[m + 1]  [4] out i32 counts[M]  [5] out i32 offsets[M + 1] (multiples of 256; offsets[M] = the
  *              padded row count)  [6] out i32 block_model[capacity / 256]: the net of each 256-row block
- * An empty batch (n_envs = 0) zeroes counts / offsets when they are given. */
+ * An empty batch (n_envs = 0) zeroes counts / offsets when they are given.
+ * BRL_F_PLAYER_MODELS: [2] is i32 env_models[n,4] by player id instead, and env i's acting net is env_models[i][player]
+ * (the two partners of a team may be different nets); the bad-id rule is the same. */
+#define BRL_F_PLAYER_MODELS (1 << 24)  /* brl_model_rows / brl_duplicate_match: a net per player id, env_models[n,4] */
 int32_t brl_model_rows(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 /* brl_policy_act_rows with the net of each row block taken from the pool (masked argmax only; BRL_F_SAMPLE is an error).
  * The row count n_rows[0] (offsets[M] of brl_model_rows, e.g. a pointer to offsets + M) is read on the device only: the call
@@ -357,7 +360,10 @@ int32_t brl_match_stats_ranges(brl_stream_t, void **buffers, const void *opaque,
  *          [9..14] out final Table_info A {u8 terminated, f32 rewards[n,4], i32 last_bid, i32 last_bidder, u8 call_x,
  *          u8 call_xx}  [15..20] out Table_info B -- all twelve or none (then they live in the scratch)
  * params: n_envs = n, k_steps = M, step = P (0 with [4] NULL), n_deals, illegal_penalty / illegal_bonus as brl_step,
- *         flags BRL_F_MLP_BF16 / BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED (BRL_F_SAMPLE is an error). */
+ *         flags BRL_F_MLP_BF16 / BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED (BRL_F_SAMPLE is an error).
+ * BRL_F_PLAYER_MODELS: [3] is a required i32 env_models[n,4] by player id (brl_model_rows' flag; NULL is BRL_E_BUFFER), so
+ * each player of a match may be a different net: partnerships of two nets (cross-play).  Player ids keep their team at both
+ * tables (table B swaps seats, not ids), so the ids need no change at the table switch. */
 #define BRL_MATCH_MAX_STEPS 638    /* an auction has at most 319 calls; an env finishes both tables in at most 638 steps */
 #define BRL_MATCH_OK 0
 #define BRL_MATCH_BAD_MODEL 1      /* a live env's acting net id is outside [0, M): the loop stopped, outputs invalid */
@@ -384,6 +390,11 @@ int32_t brl_duplicate_match(brl_stream_t, void **buffers, const void *opaque, si
  * BRL_F_EVAL_FREE_RUN (full statistics only, game_mode "free-run"): team 2 always passes.  Every live row is forwarded by net 0
  * (team 2's too: brl_model_rows needs no change) and brl_eval_act_log reads no team-2 logits, so the results equal the host
  * loop's at the cost of forwarding team 2's rows; net 1 is not read.
+ * BRL_F_EVAL_PARTNER: the pool holds 3 nets (k_steps = 3): net 0 is the actor, net 1 team 2 and net 2 the actor's partner,
+ * grouped by player id (BRL_F_PLAYER_MODELS).  DUPLICATE / SINGLE: player 0 plays net 0, player 1 net 2, players 2/3 net 1.
+ * SIMPLE: the env's initial current_player plays net 0, that player's partner net 2 and the other team net 1.  With
+ * BRL_F_EVAL_FREE_RUN team 2 still passes and net 1 is not read: team 2's rows are forwarded by net 0, team 1's are split
+ * between nets 0 and 2.  The scratch is brl_evaluate_match_partner_scratch_bytes(n, mode).
  * buffers: [0] in u64 keys[n]  [1] in deal_table  [2] in pool u8[2, brl_mlp_pool_stride()]
  *          [3] scratch (brl_evaluate_match_scratch_bytes(n, mode))  [4] out f32 cum_return[n] (simple: R[n])
  *          [5] out f32 acc[n, BRL_EVAL_ACC_COLS] (full statistics; simple: not read)
@@ -402,7 +413,9 @@ int32_t brl_duplicate_match(brl_stream_t, void **buffers, const void *opaque, si
 #define BRL_F_EVAL_MATCH(mode) ((mode) << 27)
 #define BRL_EVAL_MATCH_MODE(flags) (((flags) >> 27) & 3)
 #define BRL_F_EVAL_FREE_RUN 0x0008
+#define BRL_F_EVAL_PARTNER (1 << 25)  /* brl_evaluate_match: a 3-net pool, net 2 the actor's partner */
 int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode);
+int64_t brl_evaluate_match_partner_scratch_bytes(int64_t n_envs, int64_t mode);
 int32_t brl_evaluate_match(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
