@@ -16,7 +16,8 @@ from . import build as _build
 # B200 (1000 W), with identical device code and identical timings under gc.disable().
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
             "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped",
-            "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats")
+            "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats",
+            "brl_system_stats", "brl_system_stats_auctions")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -63,6 +64,7 @@ EVAL_MATCH_DUPLICATE, EVAL_MATCH_SINGLE, EVAL_MATCH_SIMPLE = 1, 2, 3  # brl_eval
 F_EVAL_FREE_RUN = 0x0008  # brl_evaluate_match: team 2 always passes (BRL_F_EVAL_FREE_RUN)
 F_EVAL_PARTNER = 1 << 25  # brl_evaluate_match: a 3-net pool, net 2 the actor's partner (BRL_F_EVAL_PARTNER)
 F_PLAYER_MODELS = 1 << 24  # brl_model_rows / brl_duplicate_match: env_models[n, 4] by player id (BRL_F_PLAYER_MODELS)
+SYS_CONTEXTS, SYS_COLS = 75, 96  # the bidding-system histogram hist[M, 75, 38, 96] (BRL_SYS_*)
 
 
 def f_eval_match(mode: int) -> int:

@@ -1,7 +1,7 @@
 // brl_algo.cu -- the small per-env algorithms around the environment: GAE reverse
 // scan, masked categorical (mode / Gumbel-argmax sample / log-prob), IMP reward,
 // match-statistic partial sums, transition reward gather, double-dummy par (its reward gather and match
-// statistics).  sm_100a only.
+// statistics), bidding-system histograms.  sm_100a only.
 #include <math.h>
 
 #include "common.h"
@@ -162,12 +162,17 @@ __global__ void __launch_bounds__(1024) k_team_rows(const int8_t* __restrict__ p
 // size the forward) becomes -1, so the error surfaces before any forward runs, without an extra host read.
 constexpr int kNotListed = -1, kBadModel = -2;
 template <int kStride>
+__device__ __forceinline__ int acting_model(int player, const int32_t* env_models, int64_t i, int n_models) {
+    static_assert(kStride == 2 || kStride == 4, "env_models holds a net per team or per player");
+    const int m = env_models[kStride * i + (kStride == 4 ? (player & 3) : (player < 2 ? 0 : 1))];
+    return m >= 0 && m < n_models ? m : kBadModel;
+}
+
+template <int kStride>
 __device__ __forceinline__ int acting_model(const int8_t* player, const uint8_t* done, const int32_t* env_models, int64_t i,
                                             int64_t n, int n_models) {
-    static_assert(kStride == 2 || kStride == 4, "env_models holds a net per team or per player");
     if (i >= n || (done != nullptr && done[i] != 0)) return kNotListed;
-    const int m = env_models[kStride * i + (kStride == 4 ? (player[i] & 3) : (player[i] < 2 ? 0 : 1))];
-    return m >= 0 && m < n_models ? m : kBadModel;
+    return acting_model<kStride>(player[i], env_models, i, n_models);
 }
 
 template <int kStride>
@@ -245,6 +250,50 @@ __global__ void __launch_bounds__(256) k_model_scatter(const int8_t* __restrict_
     if (m >= 0 && lane == leader) base = atomicAdd(&cursor[m], __popc(peers));
     base = __shfl_sync(0xffffffffu, base, leader);
     if (m >= 0) rows[offsets[m] + base + __popc(peers & ((1u << lane) - 1u))] = (int32_t)i;
+}
+
+// ---- bidding-system statistics (env_device.cuh, DESIGN.md f15) ---------------------------------------------------------------
+// One decision per live env, in the state before the step, into the histogram of the net acting there (acting_model, the rule
+// of brl_model_rows; no env_models: net 0).  A call outside 0..37 or a net id outside [0, M) is not counted.
+template <int kStride>
+__global__ void __launch_bounds__(256) k_system_stats(const uint4* __restrict__ state, int64_t stride, const uint8_t* __restrict__ table,
+                                                      const int32_t* __restrict__ action, const uint8_t* __restrict__ done,
+                                                      const int32_t* __restrict__ env_models, uint32_t* __restrict__ hist, int64_t n,
+                                                      int n_models) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || (done != nullptr && done[i] != 0)) return;
+    const int32_t a = action[i];
+    if (a < 0 || a >= kNumActions) return;
+    Env e;
+    load_env(state, stride, i, e);
+    const uint32_t seat = f_cur_seat(e);
+    const int m = env_models != nullptr ? acting_model<kStride>((int)f_player_at(e, seat), env_models, i, n_models) : 0;
+    if (m < 0) return;
+    system_count(hist + m * kSysCells, system_context(system_prefix(e)), (uint32_t)a, hand_features(TableRows{table}.hand(e.deal, seat)));
+}
+
+// Every call of stored auctions, one thread per auction: auction t is calls[offsets[t], offsets[t + 1]) on deal row board[t]
+// (NULL: t) with dealer dealer[t] (NULL: North).  The calls and rows are the caller's checked input.
+__global__ void __launch_bounds__(256) k_system_stats_auctions(const uint8_t* __restrict__ table, const uint8_t* __restrict__ calls,
+                                                               const int64_t* __restrict__ offsets, const int32_t* __restrict__ board,
+                                                               const int8_t* __restrict__ dealer, uint32_t* __restrict__ hist,
+                                                               int64_t n) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const uint32_t row = board != nullptr ? (uint32_t)board[t] : (uint32_t)t;
+    const uint32_t d = dealer != nullptr ? (uint32_t)dealer[t] & 3u : 0u;
+    const TableRows rows{table};
+    HandFeatures f[4];
+#pragma unroll
+    for (uint32_t s = 0; s < 4u; ++s) f[s] = hand_features(rows.hand(row, s));
+    SystemPrefix p{};
+    const int64_t end = offsets[t + 1];
+    for (int64_t k = offsets[t]; k < end; ++k) {
+        const uint32_t c = calls[k], seat = (d + p.t) & 3u;
+        const HandFeatures& h = seat == 0u ? f[0] : (seat == 1u ? f[1] : (seat == 2u ? f[2] : f[3]));
+        system_count(hist, system_context(p), c, h);
+        system_push(p, c);
+    }
 }
 
 // ---- _imp_reward -- src/duplicate.py:15-70 ----------------------------------------------------
@@ -633,6 +682,51 @@ int32_t brl_par_stats(brl_stream_t stream, void** b, const void* opaque, size_t 
         static_cast<const int32_t*>(b[3]), static_cast<const int32_t*>(b[4]), static_cast<const float*>(b[5]),
         static_cast<const int32_t*>(b[6]), static_cast<const int32_t*>(b[7]), static_cast<double*>(b[8]), p->n_envs);
     return check_launch("brl_par_stats");
+}
+
+int32_t brl_system_stats(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    if (p->k_steps <= 0) return fail(BRL_E_OPAQUE, "brl_system_stats: k_steps (the histogram's net count) must be > 0");
+    static const char* names[] = {"state", "deal_table", "action", "done", "env_models", "hist"};
+    if ((rc = check_buffers("brl_system_stats", b, names, 6, 1u << 3 | 1u << 4, 1u << 0)) != BRL_OK) return rc;
+    const bool player_models = (p->flags & BRL_F_PLAYER_MODELS) != 0;
+    if (player_models && b[4] == nullptr) return fail(BRL_E_BUFFER, "brl_system_stats: BRL_F_PLAYER_MODELS needs env_models [4] (i32[n, 4])");
+    if ((reinterpret_cast<uintptr_t>(b[2]) | reinterpret_cast<uintptr_t>(b[4]) | reinterpret_cast<uintptr_t>(b[5])) & 3u)
+        return fail(BRL_E_BUFFER, "brl_system_stats: action, env_models and hist must be 4-byte aligned");
+    const int64_t stride = p->state_stride > 0 ? p->state_stride : p->n_envs;
+    if (stride < p->n_envs) return fail(BRL_E_OPAQUE, "brl_system_stats: state_stride < n_envs");
+    const unsigned grid = (unsigned)((p->n_envs + 255) / 256);
+    const uint4* state = static_cast<const uint4*>(b[0]);
+    const uint8_t* table = static_cast<const uint8_t*>(b[1]);
+    const int32_t* action = static_cast<const int32_t*>(b[2]);
+    const uint8_t* done = static_cast<const uint8_t*>(b[3]);
+    const int32_t* env_models = static_cast<const int32_t*>(b[4]);
+    uint32_t* hist = static_cast<uint32_t*>(b[5]);
+    if (player_models)
+        k_system_stats<4><<<grid, 256, 0, (cudaStream_t)stream>>>(state, stride, table, action, done, env_models, hist, p->n_envs,
+                                                                 p->k_steps);
+    else
+        k_system_stats<2><<<grid, 256, 0, (cudaStream_t)stream>>>(state, stride, table, action, done, env_models, hist, p->n_envs,
+                                                                 p->k_steps);
+    return check_launch("brl_system_stats");
+}
+
+int32_t brl_system_stats_auctions(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // no auctions: a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    static const char* names[] = {"deal_table", "calls", "offsets", "board", "dealer", "hist"};
+    if ((rc = check_buffers("brl_system_stats_auctions", b, names, 6, 1u << 3 | 1u << 4, 1u << 0)) != BRL_OK) return rc;
+    if ((reinterpret_cast<uintptr_t>(b[2]) & 7u) || ((reinterpret_cast<uintptr_t>(b[3]) | reinterpret_cast<uintptr_t>(b[5])) & 3u))
+        return fail(BRL_E_BUFFER, "brl_system_stats_auctions: offsets must be 8-byte aligned, board and hist 4-byte aligned");
+    k_system_stats_auctions<<<(unsigned)((p->n_envs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint8_t*>(b[0]), static_cast<const uint8_t*>(b[1]), static_cast<const int64_t*>(b[2]),
+        static_cast<const int32_t*>(b[3]), static_cast<const int8_t*>(b[4]), static_cast<uint32_t*>(b[5]), p->n_envs);
+    return check_launch("brl_system_stats_auctions");
 }
 
 }  // extern "C"

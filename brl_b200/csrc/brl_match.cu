@@ -8,7 +8,7 @@
 //   init (brl_init) -> Table_info A / B (brl_state_fields) -> grouping (brl_model_rows) -> control
 //   WHILE (control said so) {
 //       [path kernel -> IF fused forward / IF per-layer forward]    the grouped forward, sized from the device count
-//       brl_duplicate_step -> cum_return += rewards[:, 0] -> grouping -> control
+//       [brl_system_stats] -> brl_duplicate_step -> cum_return += rewards[:, 0] -> grouping -> control
 //   }
 //   match sums (brl_match_stats_ranges, or brl_match_stats for one range)
 //
@@ -195,6 +195,7 @@ struct MatchPlan {
     float* logits;       // full statistics: the acting net's logits by env, for brl_eval_act_log (else NULL)
     float* acc;          // full statistics: the per-env log rows
     float* rewards_sum;  // single table: sum of the step rewards
+    uint32_t* system_hist;  // brl_duplicate_match [21]: bidding-system histogram of each decision (NULL: not counted)
     template <class T = void>
     T* at(size_t off) const { return reinterpret_cast<T*>(scratch + off); }
     int32_t* offsets() const { return at<int32_t>(L.offsets); }
@@ -339,6 +340,13 @@ static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, c
         p.n_envs = q.n;
         p.flags = q.mode == BRL_EVAL_MATCH_SINGLE ? BRL_F_EVAL_INDICATOR_BIDS : 0;
         if ((rc = brl_eval_act_log(s1, b, &p, sizeof(p)))) return rc;
+    }
+    if (q.system_hist) {  // each live env's decision, in the state before the step
+        void* b[6] = {q.state, const_cast<void*>(q.table), q.at(q.L.action), q.terminated, q.env_models, q.system_hist};
+        BrlParams p = env_params(q, q.n);
+        p.k_steps = q.M;
+        p.flags = q.player_models ? BRL_F_PLAYER_MODELS : 0;
+        if ((rc = brl_system_stats(s1, b, &p, sizeof(p)))) return rc;
     }
     if ((rc = env_step(q, s1))) return rc;
     if (q.mode == BRL_EVAL_MATCH_SIMPLE)
@@ -591,6 +599,7 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     if (given != 0 && given != 12) return fail(BRL_E_BUFFER, "brl_duplicate_match: give all twelve Table_info buffers [9..20] or none");
     if (given && ((reinterpret_cast<uintptr_t>(b[10]) | reinterpret_cast<uintptr_t>(b[16])) & 15u))
         return fail(BRL_E_BUFFER, "brl_duplicate_match: Table_info rewards are not 16-byte aligned");
+    if (misaligned(b[21], 4)) return fail(BRL_E_BUFFER, "brl_duplicate_match: the system histogram [21] is not 4-byte aligned");
 
     MatchPlan q = base_plan("brl_duplicate_match", 0, p, M, b[5]);
     q.P = P;
@@ -607,7 +616,8 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     q.default_models = b[3] == nullptr;
     q.player_models = player_models;  // the caller's env_models; the scratch keeps its [n, 2] layout
     if (!q.default_models) q.env_models = static_cast<int32_t*>(b[3]);
-    return run_match(q, (cudaStream_t)stream, p, b, 21);
+    q.system_hist = static_cast<uint32_t*>(b[21]);
+    return run_match(q, (cudaStream_t)stream, p, b, 22);
 }
 
 int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode) {

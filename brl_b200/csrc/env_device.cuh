@@ -296,6 +296,101 @@ __device__ __forceinline__ Par par_score(const Env& e, const Rows& rows) {
     return Par{root, c | (int32_t)(decl[owner][strain] << 8) | (int32_t)(doubled << 10)};
 }
 
+// ---- bidding-system statistics (not in the reference; DESIGN.md f15, restated by tests/system_ref.py) --------------------
+// A decision is one call a (0 Pass, 1 X, 2 XX, 3 + bid) of the player at seat s.  Its context depends only on the earlier
+// calls c_0 .. c_{t-1} of the auction (call k made by seat (dealer + k) mod 4):
+//   0 + t     OPEN(t)         every earlier call is Pass (t = the caller's position after the dealer)
+//   4 + b     RESPONSE(b)     the only bid so far is b, made by the caller's partner at call t - 2; call t - 1 was Pass; no X / XX
+//   39 + b    OVERCALL(b)     the only bid so far is b, made by the caller's right-hand opponent at call t - 1
+//   74        OTHER           everything else
+// The histogram hist[M, 75, 38, 96] (u32, +=) holds per net, context and call: columns 0..37 the HCP histogram, 38 + 14 suit
+// + len the suit-length histograms (clubs, diamonds, hearts, spades), 94 the balanced hands (no void or singleton, at most
+// one doubleton: 4333, 4432, 5332), 95 the decisions.  One call adds at most one to a cell per decision it counts.
+constexpr int kSysContexts = 75;
+constexpr int kSysOther = 74;
+constexpr int kSysCols = 96;
+constexpr int64_t kSysCells = (int64_t)kSysContexts * kNumActions * kSysCols;  // u32 per net
+
+// what the context needs from the calls before call t
+struct SystemPrefix {
+    uint32_t t;       // calls so far
+    uint32_t bids;    // bids so far, saturating at 2
+    uint32_t bid;     // the last bid (0..34)
+    uint32_t bid_at;  // its call index
+    uint32_t doubled; // an X or XX so far
+};
+
+__device__ __forceinline__ uint32_t system_context(const SystemPrefix& p) {
+    if (p.bids == 0u) return p.t < 4u ? p.t : (uint32_t)kSysOther;  // no bid: every earlier call is Pass
+    if (p.bids > 1u || p.doubled) return (uint32_t)kSysOther;
+    if (p.bid_at + 1u == p.t) return 39u + p.bid;                    // right-hand opponent's bid, the call just made
+    if (p.bid_at + 2u == p.t) return 4u + p.bid;                     // partner's bid, then a Pass (no bid, no X / XX since)
+    return (uint32_t)kSysOther;
+}
+
+// reader 1: the prefix from the packed state (the match loop).  The bid nibbles of the history say whether a bid below the
+// last one was made; X / XX are cleared by a bid, so with one bid they are the doubles of the whole auction, and the calls
+// after the last bid or double are pass_num passes.
+__device__ __forceinline__ SystemPrefix system_prefix(const Env& e) {
+    SystemPrefix p;
+    const uint32_t lb1 = f_lb1(e);
+    p.t = f_turn(e);
+    p.bid = lb1 - 1u;
+    p.doubled = f_x(e) | f_xx(e);
+    p.bid_at = p.t - 1u - f_pass_num(e);
+    uint32_t below = 0u;
+#pragma unroll
+    for (int b = 0; b < 35; ++b) {
+        const int bit = 4 * (2 + 3 * b);  // nibble of bid b (wb5/utils.py:36-38)
+        if ((uint32_t)b + 1u < lb1) below |= (e.H[bit >> 5] >> (bit & 31)) & 15u;
+    }
+    p.bids = lb1 == 0u ? 0u : (below ? 2u : 1u);
+    return p;
+}
+
+// reader 2: the prefix of a stored call sequence, one call at a time
+__device__ __forceinline__ void system_push(SystemPrefix& p, uint32_t call) {
+    if (call >= 3u) {
+        p.bids = p.bids < 2u ? p.bids + 1u : 2u;
+        p.bid = call - 3u;
+        p.bid_at = p.t;
+    } else if (call != 0u) {
+        p.doubled = 1u;
+    }
+    ++p.t;
+}
+
+// hand features of a 52-bit hand mask (card c = rank * 4 + suit, rank 0 = '2' .. 12 = 'A')
+struct HandFeatures {
+    uint32_t hcp, len[4], balanced;
+};
+
+__device__ __forceinline__ HandFeatures hand_features(uint64_t hand) {
+    constexpr uint64_t kSuit = 0x0001111111111111ull;  // bits 0, 4, .., 48: the 13 cards of clubs
+    HandFeatures f;
+    uint32_t shortest = 13u, doubletons = 0u;
+#pragma unroll
+    for (int s = 0; s < 4; ++s) {
+        f.len[s] = (uint32_t)__popcll(hand & (kSuit << s));
+        shortest = min(shortest, f.len[s]);
+        doubletons += f.len[s] == 2u;
+    }
+    f.hcp = (uint32_t)__popcll((hand >> 36) & 15u) + 2u * (uint32_t)__popcll((hand >> 40) & 15u) +
+            3u * (uint32_t)__popcll((hand >> 44) & 15u) + 4u * (uint32_t)__popcll((hand >> 48) & 15u);
+    f.balanced = shortest >= 2u && doubletons <= 1u;
+    return f;
+}
+
+// one decision into a net's histogram (hist_m = u32[75, 38, 96])
+__device__ __forceinline__ void system_count(uint32_t* __restrict__ hist_m, uint32_t context, uint32_t call, const HandFeatures& f) {
+    uint32_t* row = hist_m + ((size_t)context * kNumActions + call) * kSysCols;
+    atomicAdd(row + f.hcp, 1u);
+#pragma unroll
+    for (int s = 0; s < 4; ++s) atomicAdd(row + 38 + 14 * s + f.len[s], 1u);
+    if (f.balanced) atomicAdd(row + 94, 1u);
+    atomicAdd(row + 95, 1u);
+}
+
 __device__ __forceinline__ void history_set_bit(Env& e, uint32_t bit) {
     uint32_t w = bit >> 5, m = 1u << (bit & 31u);
 #pragma unroll

@@ -83,6 +83,8 @@
     X(brl_par, "iioo") \
     X(brl_gather_reward_par, "iiiiox") \
     X(brl_par_stats, "iiiiiiiix") \
+    X(brl_system_stats, "iiiiix") \
+    X(brl_system_stats_auctions, "iiiiix") \
     /* end */
 
 namespace {

@@ -238,12 +238,13 @@ class _MatchBuffers:
         v.pool, v.scratch, v.status, v.tables = self.pool, self.scratch, self.status, self.tables
         return v
 
-    def play(self, eval_env, single_bf16: bool, tune: int):
+    def play(self, eval_env, single_bf16: bool, tune: int, system_hist=None):
         self.sums.zero_()
         ops.duplicate_match(self.keys, eval_env.table, self.pool, self.scratch, self.cum_return, self.sums, self.status,
                             env_models=self.env_models, range_offsets=self.offsets, table_a=self.tables[0],
                             table_b=self.tables[1], single_bf16=single_bf16, tune=tune,
-                            illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
+                            illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus,
+                            system_hist=system_hist)
 
 
 def _check_match_status(status: int, op: str = "brl_duplicate_match") -> None:
@@ -341,7 +342,9 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
     with a caller's pool ONE set, allocated by `matches.reserve(pool, max_pairs)` for the largest chunk of up to `max_pairs`
     matches (pair_match_bytes of _pool_match_shape), every chunk playing on a prefix of it -- so a pool whose pair count grows
     call by call (a filling zoo) holds exactly that memory from the reservation on.  `cum_returns` (a dict, tests) receives
-    each pair's per-env returns of this rank's shard."""
+    each pair's per-env returns of this rank's shard.  `system_hist` (int64 [M, 75, 38, 96] on the device): every decision of
+    this rank's shard is added to the histogram of the net that made it (brl_duplicate_match [21], one u32 histogram per chunk
+    added in); the caller all-reduces it."""
     import numpy as np
     rank, world = bdist.rank_world()
     n, dev = num_eval_envs, eval_env.device
@@ -350,6 +353,7 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
     held = {}                                                   # the caller pool's set: pool, max_pairs, buffers
     blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
     single_bf16 = forward_pass.precision == "tc-bf16"
+    chunk_hists = {}                                            # M -> the u32 histogram one chunk counts into
 
     def reserve(pool, max_pairs: int) -> None:
         if held and held["pool"] is pool and held["max_pairs"] >= max_pairs:
@@ -359,7 +363,7 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
         held.update(pool=pool, max_pairs=max_pairs,
                     buffers=_MatchBuffers(n_envs, pool.shape[0], P, dev, with_models=True, with_tables=False, pool=pool))
 
-    def matches(pairs, rng_key, params_list=None, pool=None, cum_returns=None):
+    def matches(pairs, rng_key, params_list=None, pool=None, cum_returns=None, system_hist=None):
         M = len(params_list) if pool is None else pool.shape[0]
         width = len(pairs[0]) if len(pairs) else 2             # nets by team (i, j) or by player (a, b, c, d)
         if width not in (2, 4) or any(len(p) != width for p in pairs) or (width == 4 and pool is not None):
@@ -388,7 +392,15 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
                 b.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
                 b.env_models.copy_(torch.as_tensor(pair_arr[c0 + g // n], device=dev))
                 b.offsets.copy_(torch.as_tensor(bounds, device=dev))
-                b.play(eval_env, single_bf16, tune)
+                if system_hist is None:
+                    b.play(eval_env, single_bf16, tune)
+                else:
+                    if M not in chunk_hists:
+                        chunk_hists[M] = ops.new_system_hist(M, dev)
+                    chunk_hist = chunk_hists[M]
+                    chunk_hist.zero_()
+                    b.play(eval_env, single_bf16, tune, chunk_hist)
+                    system_hist += ops.system_hist_counts(chunk_hist)
                 sums[p_lo:p_hi] = b.sums
                 status = b.status
                 if cum_returns is not None:
@@ -457,6 +469,32 @@ def make_crossplay_evaluate(eval_env, activation, model_type, num_eval_envs: int
         return stats, imp
 
     return crossplay
+
+
+def make_bidding_system_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *,
+                                 tune: int = 0):
+    """The bidding systems of M nets (DESIGN.md f15): `system(params_list, rng_key, opponent=None)` returns int64
+    hist[M, 75, 38, 96] on the host, every decision of the nets' duplicate matches counted for the net that made it.  By
+    default net m plays all four seats in block m (its system as it plays with and against itself); with `opponent=k` net m
+    plays players 0/1 against net k on 2/3 (match m is `make_simple_duplicate_evaluate(...)(params_list[m],
+    params_list[k], rng_key)`), and net k's decisions in every match count for net k.  Every match is played on the same
+    boards.  The matches run on the pair-match engine (at most `max_envs` envs per rank a chunk, one brl_duplicate_match
+    call each, sharded by global env index) with one int64 all-reduce of the histogram per call, so the result does not
+    depend on the rank count.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward's path."""
+    matches = _make_device_pair_matches(eval_env, make_forward_pass(activation=activation, model_type=model_type),
+                                        num_eval_envs, max_envs, tune)
+
+    def system(params_list, rng_key, opponent=None):
+        M = len(params_list)
+        if opponent is not None and not 0 <= opponent < M:
+            raise ValueError(f"make_bidding_system_evaluate: opponent {opponent} is not a net of the {M} given")
+        pairs = [(m, m if opponent is None else opponent) for m in range(M)]
+        hist = torch.zeros((M,) + ops.SYSTEM_SHAPE, dtype=torch.int64, device=eval_env.device)
+        matches(pairs, rng_key, params_list=params_list, system_hist=hist)
+        bdist.allreduce_sums(hist)
+        return hist.cpu().numpy()
+
+    return system
 
 
 def make_device_pfsp_probe(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):

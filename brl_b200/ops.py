@@ -741,13 +741,15 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
                     sums: torch.Tensor, status: torch.Tensor, *, env_models: Optional[torch.Tensor] = None,
                     range_offsets: Optional[torch.Tensor] = None, table_a: Optional[TableInfoBuffers] = None,
                     table_b: Optional[TableInfoBuffers] = None, single_bf16: bool = False, tune: int = 0,
-                    illegal_penalty: float = -1.0, illegal_bonus: float = 1.0) -> None:
+                    illegal_penalty: float = -1.0, illegal_bonus: float = 1.0,
+                    system_hist: Optional[torch.Tensor] = None) -> None:
     """Play duplicate_evaluate's whole loop (src/evaluation.py:93-201) for every env of `keys` in one call, with the loop on
     the device: env e plays net env_models[e, 0] of `pool` on players 0/1 against env_models[e, 1] on 2/3 (default: net 0
     against net 1, M must be 2), or with env_models int32[n, 4] net env_models[e, p] on player p (BRL_F_PLAYER_MODELS: each
     partner may be a different net).  Writes cum_return f32[n], adds the match sums to `sums` (f64[P, 8] over the ranges of
     `range_offsets` int64[P + 1], or f64[8] for the whole batch), the status (int32[1], _lib.MATCH_*) and, when given, the
-    final Table_info of both tables.  Nothing is read back to the host; read `status` with the sums."""
+    final Table_info of both tables.  `system_hist` (u32 [M, 75, 38, 96], see `system_stats`): every decision of the match is
+    added to the histogram of the net that made it.  Nothing is read back to the host; read `status` with the sums."""
     n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
     if env_models is None and M != 2:
         raise _lib.BrlError(f"duplicate_match: without env_models the pool must hold 2 nets, got {M}")
@@ -769,9 +771,11 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
         raise _lib.BrlError("duplicate_match: scratch too small (ops.duplicate_match_scratch_bytes)")
     if (table_a is None) != (table_b is None):
         raise _lib.BrlError("duplicate_match: give both Table_info outputs or neither")
+    if system_hist is not None:
+        _check_system_hist("duplicate_match", system_hist, M)
     infos = table_a.ptrs() + table_b.ptrs() if table_a is not None else [None] * 12
     _call("brl_duplicate_match", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(env_models), _ptr(range_offsets), _ptr(scratch),
-                                  _ptr(cum_return), _ptr(sums), _ptr(status)] + infos,
+                                  _ptr(cum_return), _ptr(sums), _ptr(status)] + infos + [_ptr(system_hist)],
           _params(n, k_steps=M, step=P, n_deals=table.shape[0],
                   flags=(F_MLP_BF16 if single_bf16 else 0) | (_lib.F_PLAYER_MODELS if player_models else 0) | tune,
                   illegal_penalty=illegal_penalty, illegal_bonus=illegal_bonus))
@@ -834,3 +838,82 @@ def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, 
                                  _ptr(status)] + infos + finals,
           _params(n, n_deals=table.shape[0], flags=flags, k_steps=3 if partner else 0, illegal_penalty=illegal_penalty,
                   illegal_bonus=illegal_bonus))
+
+
+# ---- bidding-system statistics (DESIGN.md f15) ---------------------------------------------------------------------------
+SYSTEM_SHAPE = (_lib.SYS_CONTEXTS, NUM_ACTIONS, _lib.SYS_COLS)  # one net's histogram: [context, call, column]
+
+
+def new_system_hist(n_models: int, device) -> torch.Tensor:
+    """A zeroed bidding-system histogram u32 [M, 75, 38, 96] for `system_stats` / `duplicate_match(system_hist=)`."""
+    return torch.zeros((n_models,) + SYSTEM_SHAPE, dtype=torch.uint32, device=device)
+
+
+def system_hist_counts(hist: torch.Tensor) -> torch.Tensor:
+    """The u32 cells of a device histogram as int64 (for accumulating calls beyond 2^32 - 1)."""
+    return hist.view(torch.int32).to(torch.int64) & 0xFFFFFFFF
+
+
+def _check_system_hist(who: str, hist: torch.Tensor, n_models: int) -> None:
+    if hist.dtype not in (torch.uint32, torch.int32) or tuple(hist.shape) != (n_models,) + SYSTEM_SHAPE:
+        raise _lib.BrlError(f"{who}: the system histogram must be u32 [{n_models}, 75, 38, 96] (ops.new_system_hist)")
+
+
+def system_stats(state: torch.Tensor, table: torch.Tensor, action: torch.Tensor, hist: torch.Tensor, *,
+                 done: Optional[torch.Tensor] = None, env_models: Optional[torch.Tensor] = None) -> None:
+    """hist += one decision per live env (done == 0; no `done`: every env): the call action[i] of the player to act in
+    `state` (before the step), with that player's hand, in the context the earlier calls give it, counted for the net acting
+    there -- env_models int32 [n, 2] by team or [n, 4] by player id, as `model_rows` reads them (None: net 0).  `hist` is
+    u32 [M, 75, 38, 96]; a call outside 0..37 or a net id outside [0, M) is not counted."""
+    n = int(action.shape[0])
+    M = int(hist.shape[0]) if hist.dim() == 4 else 0
+    _check_system_hist("system_stats", hist, max(M, 1))
+    if state.dtype != torch.int32 or state.dim() != 3 or state.shape[0] != STATE_PLANES or state.shape[1] < n:
+        raise _lib.BrlError("system_stats: state must be a packed state int32 [5, >= n, 4] (ops.new_state)")
+    if action.dtype != torch.int32 or action.dim() != 1:
+        raise _lib.BrlError("system_stats: action must be int32 [n]")
+    if done is not None and (done.dtype not in (torch.uint8, torch.bool) or tuple(done.shape) != (n,)):
+        raise _lib.BrlError("system_stats: done must be uint8 / bool [n]")
+    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4))):
+        raise _lib.BrlError("system_stats: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
+        raise _lib.BrlError("system_stats: the deal table must be u8 [n_deals, 48]")
+    flags = _lib.F_PLAYER_MODELS if env_models is not None and env_models.shape[1] == 4 else 0
+    _call("brl_system_stats", [_ptr(state), _ptr(table), _ptr(action), _ptr(done), _ptr(env_models), _ptr(hist)],
+          _params(n, stride=state.shape[1], k_steps=M, n_deals=table.shape[0], flags=flags))
+
+
+def system_stats_auctions(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tensor, hist: torch.Tensor, *,
+                          board: Optional[torch.Tensor] = None, dealer: Optional[torch.Tensor] = None) -> None:
+    """hist (u32 [1, 75, 38, 96]) += every call of the stored auctions: auction t is calls[offsets[t]:offsets[t + 1]] (u8,
+    0..37, the encoding of `sl_examples`) on deal row board[t] (int32; None: row t) with dealer dealer[t] (int8; None: North).
+    The calls, the rows and the dealers are checked on the host (one device-to-host copy of each) before any device work."""
+    n = int(offsets.shape[0]) - 1
+    _check_system_hist("system_stats_auctions", hist, 1)
+    if offsets.dtype != torch.int64 or offsets.dim() != 1 or n < 0:
+        raise _lib.BrlError("system_stats_auctions: offsets must be int64 [n + 1]")
+    if calls.dtype != torch.uint8 or calls.dim() != 1:
+        raise _lib.BrlError("system_stats_auctions: calls must be u8 [total]")
+    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
+        raise _lib.BrlError("system_stats_auctions: the deal table must be u8 [n_deals, 48]")
+    if board is not None and (board.dtype != torch.int32 or tuple(board.shape) != (n,)):
+        raise _lib.BrlError("system_stats_auctions: board must be int32 [n]")
+    if dealer is not None and (dealer.dtype != torch.int8 or tuple(dealer.shape) != (n,)):
+        raise _lib.BrlError("system_stats_auctions: dealer must be int8 [n]")
+    if n == 0:
+        return
+    off = offsets.cpu()
+    if int(off[0]) != 0 or bool((off[1:] < off[:-1]).any()) or int(off[-1]) != calls.shape[0]:
+        raise _lib.BrlError("system_stats_auctions: offsets must rise from 0 to len(calls)")
+    if int(off[-1]) >= 1 << 32:
+        raise _lib.BrlError("system_stats_auctions: at most 2^32 - 1 calls per call (a u32 cell could wrap)")
+    if calls.numel() and int(calls.max()) >= NUM_ACTIONS:
+        raise _lib.BrlError("system_stats_auctions: a call is outside 0..37")
+    if board is None and n > table.shape[0]:
+        raise _lib.BrlError("system_stats_auctions: without board auction t needs deal row t: the table is too short")
+    if board is not None and (int(board.min()) < 0 or int(board.max()) >= table.shape[0]):
+        raise _lib.BrlError("system_stats_auctions: a board row is outside the deal table")
+    if dealer is not None and (int(dealer.min()) < 0 or int(dealer.max()) > 3):
+        raise _lib.BrlError("system_stats_auctions: a dealer is outside 0..3")
+    _call("brl_system_stats_auctions", [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(board), _ptr(dealer), _ptr(hist)],
+          _params(n, n_deals=table.shape[0]))

@@ -57,6 +57,8 @@
  *   brl_ppo_grad_anchored / brl_ppo_grad_grouped_anchored   brl_ppo_grad(_grouped) + a KL penalty toward a fixed anchor policy
  *   brl_par / brl_gather_reward_par / brl_par_stats   not in the reference: the double-dummy par of each board, the
  *                         transition reward as IMPs against it, and a duplicate match's bidding against it (DESIGN.md f13)
+ *   brl_system_stats / brl_system_stats_auctions   not in the reference: the hand strength and shape behind each call, by
+ *                         net, context and call, counted in the match loop or over stored auctions (DESIGN.md f15)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -359,6 +361,10 @@ int32_t brl_match_stats_ranges(brl_stream_t, void **buffers, const void *opaque,
  *          brl_match_stats_ranges; sums[8] for one range)  [8] out i32 status[1] (BRL_MATCH_*)
  *          [9..14] out final Table_info A {u8 terminated, f32 rewards[n,4], i32 last_bid, i32 last_bidder, u8 call_x,
  *          u8 call_xx}  [15..20] out Table_info B -- all twelve or none (then they live in the scratch)
+ *          [21] inout u32 system_hist[M, 75, 38, 96] (NULL: not counted): each iteration runs brl_system_stats between the
+ *          grouped forward and brl_duplicate_step, on the forward's actions and this call's env_models (by team or by player),
+ *          so every decision of the match is counted for the net that made it.  Without it the graph is the one without
+ *          the histogram.  The XLA form keeps the 21-buffer layout: [21] is NULL there.
  * params: n_envs = n, k_steps = M, step = P (0 with [4] NULL), n_deals, illegal_penalty / illegal_bonus as brl_step,
  *         flags BRL_F_MLP_BF16 / BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED (BRL_F_SAMPLE is an error).
  * BRL_F_PLAYER_MODELS: [3] is a required i32 env_models[n,4] by player id (brl_model_rows' flag; NULL is BRL_E_BUFFER), so
@@ -417,6 +423,39 @@ int32_t brl_duplicate_match(brl_stream_t, void **buffers, const void *opaque, si
 int64_t brl_evaluate_match_scratch_bytes(int64_t n_envs, int64_t mode);
 int64_t brl_evaluate_match_partner_scratch_bytes(int64_t n_envs, int64_t mode);
 int32_t brl_evaluate_match(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
+/* ---- bidding-system statistics (not in the reference; DESIGN.md f15, restated by tests/system_ref.py) --------------------
+ * A decision is one call a (BRL_NUM_ACTIONS numbering) of the player at seat s.  Its context c in [0, 75) depends only on the
+ * earlier calls of the auction (call k made by seat (dealer + k) mod 4):
+ *   c = t        OPEN(t), t = 0..3: every earlier call is Pass (t = the caller's position after the dealer)
+ *   c = 4 + b    RESPONSE(b): the only bid so far is bid b (0..34), made by the caller's partner two calls ago; the call since
+ *                was Pass; no X / XX
+ *   c = 39 + b   OVERCALL(b): the only bid so far is bid b, made by the caller's right-hand opponent at the previous call
+ *   c = 74       OTHER
+ * Hand features of seat s from the deal row: HCP (A 4, K 3, Q 2, J 1; 0..37), suit lengths (clubs, diamonds, hearts,
+ * spades), balanced = no void or singleton and at most one doubleton (4333, 4432, 5332).
+ * hist[M, 75, 38, 96] u32 (+=), per net m, context c and call a: columns 0..37 the HCP histogram, 38 + 14 * suit + length the
+ * suit-length histograms, 94 the balanced hands, 95 the decisions (1,094,400 bytes per net).  A call adds one to at most seven
+ * cells per decision it counts, so a cell stays exact while hist plus the call's decisions stays below 2^32; callers that
+ * accumulate longer add each call's histogram into a wider one. */
+#define BRL_SYS_CONTEXTS 75
+#define BRL_SYS_COLS 96
+/* One decision per live env, in the state before the step: the call action[i] of the player to act, into the histogram of the
+ * net acting there by brl_model_rows' rule (env_models by team, or by player with BRL_F_PLAYER_MODELS; NULL: net 0 for every
+ * env).  Calls outside 0..37 and net ids outside [0, M) are not counted.  One thread per env, global atomics into the
+ * (L2-resident) histogram.
+ * buffers: [0] in state (16-byte aligned)  [1] in deal_table  [2] in i32 action[n]  [3] in u8 done[n] (NULL: all live)
+ *          [4] in i32 env_models[n, 2] by team or [n, 4] by player id with BRL_F_PLAYER_MODELS (NULL: net 0)
+ *          [5] inout u32 hist[M, 75, 38, 96]
+ * params: n_envs, state_stride (0: n_envs), k_steps = M, flags BRL_F_PLAYER_MODELS. */
+int32_t brl_system_stats(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* Every call of stored auctions, the context read from the call sequence (no env replay): auction t is calls[offsets[t],
+ * offsets[t + 1]) (brl_sl_examples' encoding) on deal row board[t] with dealer dealer[t].  Calls must be in 0..37 and rows in
+ * the table: they are not checked here.
+ * buffers: [0] in deal_table  [1] in u8 calls[]  [2] in i64 offsets[n + 1]  [3] in i32 board[n] (NULL: row t)
+ *          [4] in i8 dealer[n] (NULL: North, the convention of the OpenSpiel data files)  [5] inout u32 hist[1, 75, 38, 96]
+ * params: n_envs = n auctions. */
+int32_t brl_system_stats_auctions(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
@@ -678,6 +717,8 @@ void brl_sl_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t op
 void brl_sl_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_gather_reward_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_system_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_system_stats_auctions_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------

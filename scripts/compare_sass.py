@@ -8,9 +8,8 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the per-player nets of partnerships: k_model_count and k_model_scatter become templates on the
-env_models stride, their per-team instantiation <2> the kernel they were; <4> (BRL_F_PLAYER_MODELS), k_player_models and
-k_actor_partner_models (BRL_F_EVAL_PARTNER) are new.  Replace both tables for another change."""
+RENAMES and ADDED record the bidding-system statistics: no kernel is renamed, and k_system_stats (per team <2> and per
+player <4>) and k_system_stats_auctions are new.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -18,9 +17,8 @@ import subprocess
 import sys
 from collections import OrderedDict
 
-RENAMES = [(r"^brl::k_model_count$", "brl::k_model_count<(int)2>"), (r"^brl::k_model_scatter$", "brl::k_model_scatter<(int)2>")]  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-ADDED = [r"^brl::k_model_count<\(int\)4>$", r"^brl::k_model_scatter<\(int\)4>$", r"^brl::k_player_models$",
-         r"^brl::k_actor_partner_models$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
+RENAMES = []  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
+ADDED = [r"^brl::k_system_stats<\(int\)2>$", r"^brl::k_system_stats<\(int\)4>$", r"^brl::k_system_stats_auctions$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):
