@@ -17,7 +17,7 @@ from . import build as _build
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
             "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped",
             "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats",
-            "brl_system_stats", "brl_system_stats_auctions")
+            "brl_system_stats", "brl_system_stats_auctions", "brl_call_values")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -35,7 +35,7 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes",
         "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes",
         "brl_evaluate_match_partner_scratch_bytes",
-        "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride")
+        "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride", "brl_call_values_scratch_bytes")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 
@@ -58,7 +58,7 @@ F_COUNT_DONE = 0x8000
 ABI_VERSION = 3  # include/brl_b200.h BRL_ABI_VERSION; load() refuses a library built from other headers
 EVAL_ACC_COLS = 76
 MATCH_MAX_STEPS = 638  # brl_duplicate_match's bound on forwards (BRL_MATCH_MAX_STEPS)
-MATCH_OK, MATCH_BAD_MODEL, MATCH_STEP_BOUND = 0, 1, 2  # its status codes (BRL_MATCH_*)
+MATCH_OK, MATCH_BAD_MODEL, MATCH_STEP_BOUND, MATCH_RECORD_CAPACITY = 0, 1, 2, 3  # its status codes (BRL_MATCH_*)
 F_TUNE_MLP_LAYERS, F_TUNE_MLP_FUSED = 1 << 29, 1 << 30  # pin the policy forward's path (BRL_F_TUNE_MLP_*)
 EVAL_MATCH_DUPLICATE, EVAL_MATCH_SINGLE, EVAL_MATCH_SIMPLE = 1, 2, 3  # brl_evaluate_match's modes (BRL_EVAL_MATCH_*)
 F_EVAL_FREE_RUN = 0x0008  # brl_evaluate_match: team 2 always passes (BRL_F_EVAL_FREE_RUN)

@@ -4,6 +4,8 @@
 //   brl_evaluate_match    make_evaluate's duplicate / single-table evaluate (:207-1032) and make_simple_evaluate (:11-66):
 //                         the same loop with the step log (brl_eval_act_log) and the statistics (brl_eval_summary), or with
 //                         one env step per iteration and the actor's return
+//   brl_call_values       brl_duplicate_match's loop with, after each forward, every live env branched on every legal call and
+//                         the branches played out by a nested WHILE node (DESIGN.md f16)
 //
 //   init (brl_init) -> Table_info A / B (brl_state_fields) -> grouping (brl_model_rows) -> control
 //   WHILE (control said so) {
@@ -30,6 +32,7 @@
 #include <string>
 
 #include "common.h"
+#include "env_device.cuh"
 
 namespace brl {
 
@@ -118,6 +121,109 @@ __global__ void k_match_path(const int32_t* __restrict__ n_rows, cudaGraphCondit
     const bool f = *n_rows >= kPairMinM;
     cudaGraphSetConditional(fused, f ? 1u : 0u);
     cudaGraphSetConditional(layers, f ? 0u : 1u);
+}
+
+// ---- brl_call_values (env_device.cuh, DESIGN.md f16) ----------------------------------------------------------------------
+// the loop condition of brl_call_values' two loops: like k_match_control with the bound a parameter, and a stop once a loop
+// has failed (a BRL_MATCH_RECORD_CAPACITY status does not stop the loops: the sums stay complete)
+__global__ void k_cv_control(const int32_t* __restrict__ n_rows, int32_t* __restrict__ iter, int32_t* __restrict__ status,
+                             cudaGraphConditionalHandle loop, int bound) {
+    const int rows = *n_rows, it = *iter, st = *status;
+    bool go = rows > 0 && st != BRL_MATCH_BAD_MODEL && st != BRL_MATCH_STEP_BOUND;
+    if (rows < 0) {
+        *status = BRL_MATCH_BAD_MODEL;
+    } else if (go && it >= bound) {
+        *status = BRL_MATCH_STEP_BOUND;
+        go = false;
+    }
+    if (go) *iter = it + 1;
+    cudaGraphSetConditional(loop, go ? 1u : 0u);
+}
+
+// one thread per branch slot j = 38 i + a of base env i: the slot's state is S_i, to be stepped with call a by brl_step; a
+// slot whose env is finished or whose call is illegal is born finished (a no-op step, never listed by brl_model_rows).  The
+// slot's nets by player id come from the env's (by team: expanded); r[j] = 0; the slot loop's iteration counter restarts.
+template <int kStride>
+__global__ void __launch_bounds__(256) k_branch_calls(const uint4* __restrict__ state, const uint8_t* __restrict__ done,
+                                                      const int32_t* __restrict__ env_models, uint4* __restrict__ br_state,
+                                                      int32_t* __restrict__ br_action, int4* __restrict__ br_models,
+                                                      float* __restrict__ r, int32_t* __restrict__ br_iter, int64_t n) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nb = n * kNumActions;
+    if (j == 0) *br_iter = 0;
+    if (j >= nb) return;
+    const int64_t i = j / kNumActions;
+    const int a = (int)(j - i * kNumActions);
+    Env e;
+    load_env(state, n, i, e);
+    if (done[i] != 0 || !((env_legal_mask(e) >> a) & 1ull)) e.A |= kTermBit;
+    store_env(br_state, nb, j, e);
+    br_action[j] = a;
+    r[j] = 0.0f;
+    const int32_t* m = env_models + kStride * i;
+    br_models[j] = kStride == 4 ? make_int4(m[0], m[1], m[2], m[3]) : make_int4(m[0], m[0], m[1], m[1]);
+}
+
+// One thread per live base env after its branches ended: the decision's gains and regret into the int64 sums of its net,
+// context and played call (integer atomics: exact and order-independent), the invariant r(played) = R_T, and a record.
+struct CvOut {
+    unsigned long long *gain, *regret, *mismatch, *count;  // gain_sums[M,75,38,38,4], regret_sums[M,75,4], mismatch[M], count[1]
+    int32_t *env, *table, *player, *net, *context, *played;  // records (NULL: none)
+    float* r;                                                // records' r[cap, 38]
+    int64_t cap, env_offset;
+    int32_t* status;
+};
+
+template <int kStride>
+__global__ void __launch_bounds__(256) k_call_value_gains(const uint4* __restrict__ state, const uint8_t* __restrict__ done,
+                                                          const int32_t* __restrict__ env_models, const int32_t* __restrict__ action,
+                                                          const uint8_t* __restrict__ a_done, const float4* __restrict__ ra,
+                                                          const float4* __restrict__ rb, const float* __restrict__ r, CvOut o,
+                                                          int64_t n, int n_models) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || done[i] != 0) return;
+    Env e;
+    load_env(state, n, i, e);
+    const uint32_t p = f_player_at(e, f_cur_seat(e));
+    const int m = env_models[kStride * i + (kStride == 4 ? (int)p : (p < 2u ? 0 : 1))];
+    const int b = action[i];
+    if (m < 0 || m >= n_models || b < 0 || b >= kNumActions) return;
+    const uint32_t c = system_context(system_prefix(e));
+    const uint64_t legal = env_legal_mask(e);
+    const int t = a_done[i] != 0;  // table A has ended: this is table B
+    const float R_a = ra[i].x, R_b = rb[i].x, R_other = t ? R_a : R_b;
+    const float base = imp_of_difference(R_a + R_b);
+    const float* ri = r + i * kNumActions;
+    unsigned long long* gm = o.gain + (((size_t)m * kSysContexts + c) * kNumActions + b) * kNumActions * kCvStats;
+    int32_t regret = INT32_MIN;
+    for (int a = 0; a < kNumActions; ++a) {
+        if (!((legal >> a) & 1ull)) continue;
+        const long long g = call_value_gain(ri[a], R_other, base, p < 2u);
+        regret = max(regret, (int32_t)g);
+        unsigned long long* cell = gm + a * kCvStats;
+        atomicAdd(cell, 1ull);
+        atomicAdd(cell + 1, (unsigned long long)g);
+        atomicAdd(cell + 2, (unsigned long long)(g * g));
+        if (g > 0) atomicAdd(cell + 3, 1ull);
+    }
+    unsigned long long* rg = o.regret + ((size_t)m * kSysContexts + c) * kCvStats;
+    atomicAdd(rg, 1ull);
+    atomicAdd(rg + 1, (unsigned long long)(long long)regret);
+    atomicAdd(rg + 2, (unsigned long long)((long long)regret * regret));
+    if (regret > 0) atomicAdd(rg + 3, 1ull);
+    if (ri[b] != (t ? R_b : R_a)) atomicAdd(o.mismatch + m, 1ull);
+    if (o.env == nullptr) return;
+    const unsigned long long k = atomicAdd(o.count, 1ull);
+    if ((long long)k >= o.cap) {
+        atomicCAS(o.status, BRL_MATCH_OK, BRL_MATCH_RECORD_CAPACITY);
+        return;
+    }
+    o.env[k] = (int32_t)(o.env_offset + i);
+    o.table[k] = t;
+    o.player[k] = (int32_t)p;
+    o.net[k] = m;
+    o.context[k] = (int32_t)c;
+    o.played[k] = b;
+    for (int a = 0; a < kNumActions; ++a) o.r[k * kNumActions + a] = (legal >> a) & 1ull ? ri[a] : __int_as_float(0x7fc00000);
 }
 
 // ---- the scratch ----------------------------------------------------------------------------------------------------------
@@ -315,24 +421,26 @@ static int32_t env_step(const MatchPlan& q, cudaStream_t s) {
 
 // one iteration of the loop (src/evaluation.py:124-169; :388-411 / :748-777 with the step log; :42-61), on the body's capture
 // stream s1; s2 captures the IF bodies
-static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, cudaGraphConditionalHandle loop) {
+// the grouped forward of one iteration on s1: the pinned path, or the path kernel and an IF node per path (bodies captured on s2)
+static int32_t emit_forward(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2) {
+    if (q.flags & BRL_F_TUNE_MLP_LAYERS) return forward(q, s1, BRL_F_TUNE_MLP_LAYERS);
+    if (q.flags & BRL_F_TUNE_MLP_FUSED) return forward(q, s1, BRL_F_TUNE_MLP_FUSED);
     int32_t rc;
-    if (q.flags & BRL_F_TUNE_MLP_LAYERS) {
-        rc = forward(q, s1, BRL_F_TUNE_MLP_LAYERS);
-    } else if (q.flags & BRL_F_TUNE_MLP_FUSED) {
-        rc = forward(q, s1, BRL_F_TUNE_MLP_FUSED);
-    } else {
-        cudaGraphConditionalHandle h_fused, h_layers;
-        if ((rc = new_handle(q.who, s1, &h_fused)) || (rc = new_handle(q.who, s1, &h_layers))) return rc;
-        k_match_path<<<1, 1, 0, s1>>>(q.offsets() + q.M, h_fused, h_layers);
-        if ((rc = launched(q.who, "path"))) return rc;
-        cudaGraph_t body;
-        if ((rc = add_conditional(q.who, s1, h_fused, cudaGraphCondTypeIf, &body)) ||
-            (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_FUSED); })) ||
-            (rc = add_conditional(q.who, s1, h_layers, cudaGraphCondTypeIf, &body)) ||
-            (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_LAYERS); })))
-            return rc;
-    }
+    cudaGraphConditionalHandle h_fused, h_layers;
+    if ((rc = new_handle(q.who, s1, &h_fused)) || (rc = new_handle(q.who, s1, &h_layers))) return rc;
+    k_match_path<<<1, 1, 0, s1>>>(q.offsets() + q.M, h_fused, h_layers);
+    if ((rc = launched(q.who, "path"))) return rc;
+    cudaGraph_t body;
+    if ((rc = add_conditional(q.who, s1, h_fused, cudaGraphCondTypeIf, &body)) ||
+        (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_FUSED); })) ||
+        (rc = add_conditional(q.who, s1, h_layers, cudaGraphCondTypeIf, &body)) ||
+        (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) { return forward(q, s, BRL_F_TUNE_MLP_LAYERS); })))
+        return rc;
+    return BRL_OK;
+}
+
+static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, cudaGraphConditionalHandle loop) {
+    int32_t rc = emit_forward(q, s1, s2);
     if (rc != BRL_OK) return rc;
     if (q.acc) {  // the acting team's masked argmax and update_log_info; free-run: team 2 passes, its forwarded rows unread
         void* b[7] = {q.logits, q.free_run ? nullptr : q.logits, q.mask, q.player, q.terminated, q.at(q.L.action), q.acc};
@@ -460,7 +568,7 @@ static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, 
 struct MatchCache {
     std::mutex mu;
     std::map<std::string, std::pair<cudaGraphExec_t, uint64_t>> exec;  // key -> (instantiated graph, last use)
-    cudaStream_t streams[kMaxDevices][3] = {};
+    cudaStream_t streams[kMaxDevices][4] = {};
     uint64_t clock = 0;
     long long builds = 0;
 };
@@ -472,42 +580,44 @@ constexpr size_t kMaxCachedGraphs = 16;
 
 static int32_t capture_streams(const char* who, cudaStream_t** out) {
     cudaStream_t* s = cache().streams[device_slot()];
-    for (int k = 0; k < 3; ++k)
+    for (int k = 0; k < 4; ++k)
         if (s[k] == nullptr && cudaStreamCreateWithFlags(&s[k], cudaStreamNonBlocking) != cudaSuccess)
             return launched(who, "capture stream");
     *out = s;
     return BRL_OK;
 }
 
-// run plan q on `stream`: into the caller's capture when the stream is being captured, else by (building and caching, keyed by
-// the op's params and its n_buffers buffer addresses, then) launching the match's graph
-static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p, void** b, int n_buffers) {
+// run what `emit(s0, s1, s2)` enqueues on `stream`: into the caller's capture when the stream is being captured, else by
+// (building and caching, keyed by the op, its params and its n_buffers buffer addresses, then) launching its graph
+template <class Emit>
+static int32_t run_graph(const char* who, cudaStream_t s, const BrlParams* p, void** b, int n_buffers, Emit&& emit) {
     int32_t rc;
     cudaStreamCaptureStatus st;
-    if (cudaStreamIsCapturing(s, &st) != cudaSuccess) return launched(q.who, "capture status");
+    if (cudaStreamIsCapturing(s, &st) != cudaSuccess) return launched(who, "capture status");
     MatchCache& c = cache();
     std::lock_guard<std::mutex> lock(c.mu);
     cudaStream_t* side = nullptr;
-    if ((rc = warm_policy_grouped(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(q.who, &side))) return rc;
+    if ((rc = warm_policy_grouped(!(p->flags & BRL_F_MLP_BF16))) || (rc = capture_streams(who, &side))) return rc;
     if (st == cudaStreamCaptureStatusActive) {  // the caller's capture: the nodes go there
-        if ((rc = emit_match(q, s, side[1], side[2]))) return rc;
-        return check_launch(q.who);
+        if ((rc = emit(s, side))) return rc;
+        return check_launch(who);
     }
-    if (st != cudaStreamCaptureStatusNone) return fail(BRL_E_LAUNCH, "%s: the stream's capture was invalidated", q.who);
+    if (st != cudaStreamCaptureStatusNone) return fail(BRL_E_LAUNCH, "%s: the stream's capture was invalidated", who);
     int dev = 0;
     cudaGetDevice(&dev);
-    std::string key(reinterpret_cast<const char*>(&dev), sizeof(dev));
+    std::string key(who);
+    key.append(reinterpret_cast<const char*>(&dev), sizeof(dev));
     key.append(reinterpret_cast<const char*>(p), sizeof(*p));
     key.append(reinterpret_cast<const char*>(b), n_buffers * sizeof(void*));
     auto it = c.exec.find(key);
     if (it == c.exec.end()) {
-        if (cudaStreamBeginCapture(side[0], cudaStreamCaptureModeRelaxed) != cudaSuccess) return launch_error(q.who, "capture");
-        rc = emit_match(q, side[0], side[1], side[2]);
+        if (cudaStreamBeginCapture(side[0], cudaStreamCaptureModeRelaxed) != cudaSuccess) return launch_error(who, "capture");
+        rc = emit(side[0], side);
         cudaGraph_t g = nullptr;
         const cudaError_t end = cudaStreamEndCapture(side[0], &g);
         cudaGraphExec_t exec = nullptr;
         if (rc == BRL_OK && (end != cudaSuccess || cudaGraphInstantiate(&exec, g, 0) != cudaSuccess))
-            rc = launch_error(q.who, "instantiate");
+            rc = launch_error(who, "instantiate");
         if (g != nullptr) cudaGraphDestroy(g);
         if (rc != BRL_OK) return rc;
         if (c.exec.size() >= kMaxCachedGraphs) {  // evict the least recently used (a graph still running is freed when it ends)
@@ -521,8 +631,14 @@ static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p,
         ++c.builds;
     }
     it->second.second = ++c.clock;
-    if (cudaGraphLaunch(it->second.first, s) != cudaSuccess) return launched(q.who, "launch");
-    return check_launch(q.who);
+    if (cudaGraphLaunch(it->second.first, s) != cudaSuccess) return launched(who, "launch");
+    return check_launch(who);
+}
+
+static int32_t run_match(const MatchPlan& q, cudaStream_t s, const BrlParams* p, void** b, int n_buffers) {
+    return run_graph(q.who, s, p, b, n_buffers, [&](cudaStream_t s0, cudaStream_t* side) {
+        return emit_match(q, s0, side[1], side[2]);
+    });
 }
 
 // the plan's fields every mode shares; the env buffers and Table_infos start in the scratch
@@ -552,6 +668,110 @@ static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_
 }
 
 static bool misaligned(const void* ptr, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(ptr) & (bytes - 1)) != 0; }
+
+// ---- brl_call_values ----------------------------------------------------------------------------------------------------
+constexpr int kAuctionMaxCalls = BRL_MATCH_MAX_STEPS / 2;  // the bound of one branch's auction
+
+// the scratch: the base match's pieces, then a branch batch of 38 n slots (brl_duplicate_match's pieces for 38 n envs with
+// nets by player id), then the slots' r
+static size_t cv_branch_at(int64_t n, int64_t M) { return match_layout(n, M).total; }
+static size_t cv_r_at(int64_t n, int64_t M) { return cv_branch_at(n, M) + match_layout(n * kNumActions, M, 0, true).total; }
+static size_t cv_scratch_bytes(int64_t n, int64_t M) { return cv_r_at(n, M) + (size_t)n * kNumActions * 4; }
+
+struct CvPlan {
+    MatchPlan q, br;  // the base match (its Table_infos in the scratch) and the branch batch
+    const float4 *ra, *rb;
+    float* r;
+    CvOut o;
+};
+
+// brl_step without auto-reset on the branch batch, then r += rewards[:, 0] (non-zero on a slot's last step only)
+static int32_t branch_step(const CvPlan& c, cudaStream_t s) {
+    const MatchPlan& br = c.br;
+    const BrlParams p = env_params(br, br.n);
+    void* b[10] = {br.state, br.at(br.L.action), const_cast<void*>(br.table), br.state, br.obs, br.mask, br.at(br.L.rewards),
+                   br.terminated, br.player, nullptr};
+    int32_t rc;
+    if ((rc = brl_step(s, b, &p, sizeof(p)))) return rc;
+    k_add_reward<<<blocks(br.n), 256, 0, s>>>(c.r, br.at<float4>(br.L.rewards), br.n);
+    return launched(br.who, "branch reward");
+}
+
+static int32_t cv_control(const MatchPlan& q, cudaStream_t s, cudaGraphConditionalHandle loop, int bound) {
+    k_cv_control<<<1, 1, 0, s>>>(q.offsets() + q.M, q.at<int32_t>(q.L.ctl), q.status, loop, bound);
+    return launched(q.who, "control");
+}
+
+// one base iteration: forward -> branch every live env on every legal call -> play the branches out (nested WHILE) -> gains
+// -> brl_duplicate_step -> grouping -> control
+static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, cudaStream_t s3, cudaGraphConditionalHandle loop) {
+    const MatchPlan &q = c.q, &br = c.br;
+    int32_t rc;
+    if ((rc = emit_forward(q, s1, s2))) return rc;
+    const uint4* state = static_cast<const uint4*>(q.state);
+    const uint8_t* done = static_cast<const uint8_t*>(q.terminated);
+    if (q.player_models)
+        k_branch_calls<4><<<blocks(br.n), 256, 0, s1>>>(state, done, q.env_models, static_cast<uint4*>(br.state), br.at<int32_t>(br.L.action),
+                                                       reinterpret_cast<int4*>(br.env_models), c.r, br.at<int32_t>(br.L.ctl), q.n);
+    else
+        k_branch_calls<2><<<blocks(br.n), 256, 0, s1>>>(state, done, q.env_models, static_cast<uint4*>(br.state), br.at<int32_t>(br.L.action),
+                                                       reinterpret_cast<int4*>(br.env_models), c.r, br.at<int32_t>(br.L.ctl), q.n);
+    cudaGraphConditionalHandle inner;
+    if ((rc = launched(q.who, "branch calls")) || (rc = branch_step(c, s1)) || (rc = model_rows(br, s1)) ||
+        (rc = new_handle(q.who, s1, &inner)) || (rc = cv_control(br, s1, inner, kAuctionMaxCalls)))
+        return rc;
+    // the branches' auctions to their ends: the forward's IF nodes sit one level deeper here, in the nested WHILE's body
+    cudaGraph_t body;
+    if ((rc = add_conditional(q.who, s1, inner, cudaGraphCondTypeWhile, &body)) ||
+        (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) {
+             int32_t r2;
+             if ((r2 = emit_forward(br, s, s3)) || (r2 = branch_step(c, s)) || (r2 = model_rows(br, s))) return r2;
+             return cv_control(br, s, inner, kAuctionMaxCalls);
+         })))
+        return rc;
+    const int32_t* action = q.at<int32_t>(q.L.action);
+    const uint8_t* a_done = static_cast<const uint8_t*>(q.info[0][0]);
+    if (q.player_models)
+        k_call_value_gains<4><<<blocks(q.n), 256, 0, s1>>>(state, done, q.env_models, action, a_done, c.ra, c.rb, c.r, c.o, q.n, q.M);
+    else
+        k_call_value_gains<2><<<blocks(q.n), 256, 0, s1>>>(state, done, q.env_models, action, a_done, c.ra, c.rb, c.r, c.o, q.n, q.M);
+    if ((rc = launched(q.who, "gains")) || (rc = env_step(q, s1)) || (rc = model_rows(q, s1))) return rc;
+    return cv_control(q, s1, loop, BRL_MATCH_MAX_STEPS);
+}
+
+// the whole op on s0: zeroed outputs, init and Table_info A = B as brl_duplicate_match, then the base loop
+static int32_t emit_call_values(const CvPlan& c, cudaStream_t s0, cudaStream_t s1, cudaStream_t s2, cudaStream_t s3) {
+    const MatchPlan& q = c.q;
+    const size_t un = (size_t)q.n, cells = (size_t)q.M * kSysContexts * kNumActions * kNumActions * kCvStats * 8;
+    int32_t rc;
+    cudaGraphConditionalHandle loop;
+    if ((rc = new_handle(q.who, s0, &loop))) return rc;
+    if (cudaMemsetAsync(q.status, 0, sizeof(int32_t), s0) != cudaSuccess ||
+        cudaMemsetAsync(q.at(q.L.ctl), 0, sizeof(int32_t), s0) != cudaSuccess ||
+        cudaMemsetAsync(q.at(q.L.action), 0, un * sizeof(int32_t), s0) != cudaSuccess ||
+        cudaMemsetAsync(c.o.gain, 0, cells, s0) != cudaSuccess ||
+        cudaMemsetAsync(c.o.regret, 0, (size_t)q.M * kSysContexts * kCvStats * 8, s0) != cudaSuccess ||
+        cudaMemsetAsync(c.o.mismatch, 0, (size_t)q.M * 8, s0) != cudaSuccess ||
+        (c.o.count && cudaMemsetAsync(c.o.count, 0, 8, s0) != cudaSuccess))
+        return launched(q.who, "memset");
+    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
+                   q.player};
+    BrlParams p = env_params(q, q.n);
+    if ((rc = brl_init(s0, bi, &p, sizeof(p)))) return rc;
+    void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
+    if ((rc = brl_state_fields(s0, bf, &p, sizeof(p)))) return rc;
+    const size_t bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
+    if (cudaMemcpyAsync(q.info[0][0], q.terminated, bytes[0], cudaMemcpyDeviceToDevice, s0) != cudaSuccess ||
+        cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
+        return launched(q.who, "Table_info");
+    for (int k = 0; k < 6; ++k)
+        if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
+            return launched(q.who, "Table_info");
+    if ((rc = model_rows(q, s0)) || (rc = cv_control(q, s0, loop, BRL_MATCH_MAX_STEPS))) return rc;
+    cudaGraph_t body;
+    if ((rc = add_conditional(q.who, s0, loop, cudaGraphCondTypeWhile, &body))) return rc;
+    return capture_into(q.who, body, s1, [&](cudaStream_t s) { return emit_cv_body(c, s, s2, s3, loop); });
+}
 
 }  // namespace brl
 
@@ -697,6 +917,77 @@ int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, si
         }
     }
     return run_match(q, (cudaStream_t)stream, p, b, 26);
+}
+
+}  // extern "C"
+
+extern "C" {
+
+int64_t brl_call_values_scratch_bytes(int64_t n_envs, int64_t n_models) {
+    if (n_envs <= 0 || n_models <= 0) return 0;
+    return (int64_t)cv_scratch_bytes(n_envs, n_models);
+}
+
+int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_t len) {
+    int32_t rc;
+    const BrlParams* p = get_params(opaque, len, &rc);
+    if (!p) return rc;
+    if (p->n_envs == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL (zero-size XLA / torch buffers)
+    const int64_t M = p->k_steps, cap = (int64_t)p->seed;
+    const bool player_models = (p->flags & BRL_F_PLAYER_MODELS) != 0;
+    if (M <= 0) return fail(BRL_E_OPAQUE, "brl_call_values: k_steps (the pool's model count) must be > 0");
+    if (p->n_envs > INT32_MAX / 2 / kNumActions) return fail(BRL_E_OPAQUE, "brl_call_values: n_envs too large");
+    if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_call_values: n_deals must be > 0");
+    if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_call_values: sampling is not supported (argmax only)");
+    if (cap < 0) return fail(BRL_E_OPAQUE, "brl_call_values: the record capacity (seed) must be >= 0");
+    static const char* names[] = {"keys", "deal_table", "pool", "env_models", "rewards_a", "rewards_b", "scratch", "gain_sums",
+                                  "regret_sums", "mismatch", "status"};
+    if ((rc = check_buffers("brl_call_values", b, names, 11, 0u, 1u << 0 | 1u << 2 | 1u << 4 | 1u << 5 | 1u << 6)) != BRL_OK) return rc;
+    if (misaligned(b[3], 16) || misaligned(b[7], 8) || misaligned(b[8], 8) || misaligned(b[9], 8) || misaligned(b[10], 4))
+        return fail(BRL_E_BUFFER, "brl_call_values: env_models must be 16-byte, the sums 8-byte and status 4-byte aligned");
+    int given = 0;
+    for (int k = 11; k < 19; ++k) given += b[k] != nullptr;
+    if (given != 0 && given != 8) return fail(BRL_E_BUFFER, "brl_call_values: give all eight record buffers [11..18] or none");
+    if (given && (misaligned(b[11], 8) || misaligned(b[12], 4) || misaligned(b[13], 4) || misaligned(b[14], 4) ||
+                  misaligned(b[15], 4) || misaligned(b[16], 4) || misaligned(b[17], 4) || misaligned(b[18], 4)))
+        return fail(BRL_E_BUFFER, "brl_call_values: the record count must be 8-byte and the records 4-byte aligned");
+
+    CvPlan c{};
+    c.q = base_plan("brl_call_values", 0, p, M, b[6]);
+    c.q.keys = b[0];
+    c.q.table = b[1];
+    c.q.pool = static_cast<const unsigned char*>(b[2]);
+    c.q.player_models = player_models;
+    c.q.env_models = static_cast<int32_t*>(b[3]);
+    c.q.status = static_cast<int32_t*>(b[10]);
+    BrlParams pb = *p;
+    pb.n_envs = p->n_envs * kNumActions;
+    c.br = base_plan("brl_call_values", 0, &pb, M, static_cast<unsigned char*>(b[6]) + cv_branch_at(p->n_envs, M), true);
+    c.br.table = b[1];
+    c.br.pool = c.q.pool;
+    c.br.status = c.q.status;
+    c.ra = static_cast<const float4*>(b[4]);
+    c.rb = static_cast<const float4*>(b[5]);
+    c.r = reinterpret_cast<float*>(static_cast<unsigned char*>(b[6]) + cv_r_at(p->n_envs, M));
+    c.o.gain = static_cast<unsigned long long*>(b[7]);
+    c.o.regret = static_cast<unsigned long long*>(b[8]);
+    c.o.mismatch = static_cast<unsigned long long*>(b[9]);
+    c.o.status = c.q.status;
+    c.o.cap = cap;
+    c.o.env_offset = p->env_offset;
+    if (given) {
+        c.o.count = static_cast<unsigned long long*>(b[11]);
+        c.o.env = static_cast<int32_t*>(b[12]);
+        c.o.table = static_cast<int32_t*>(b[13]);
+        c.o.player = static_cast<int32_t*>(b[14]);
+        c.o.net = static_cast<int32_t*>(b[15]);
+        c.o.context = static_cast<int32_t*>(b[16]);
+        c.o.played = static_cast<int32_t*>(b[17]);
+        c.o.r = static_cast<float*>(b[18]);
+    }
+    return run_graph(c.q.who, (cudaStream_t)stream, p, b, 19, [&](cudaStream_t s0, cudaStream_t* side) {
+        return emit_call_values(c, s0, side[1], side[2], side[3]);
+    });
 }
 
 }  // extern "C"

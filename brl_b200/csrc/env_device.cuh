@@ -391,6 +391,21 @@ __device__ __forceinline__ void system_count(uint32_t* __restrict__ hist_m, uint
     atomicAdd(row + 95, 1u);
 }
 
+// ---- counterfactual call values (not in the reference; DESIGN.md f16, restated by tests/call_values_ref.py) ---------------
+// A decision d is a step of a duplicate match's env at table T (A or B) in state S_d: player p (net m by brl_model_rows'
+// rule) makes call b_d in context c = system_context(system_prefix(S_d)).  For every call a legal in S_d the branch (d, a)
+// steps S_d with a (no auto-reset, no table switch) and plays that one table to its end, every player acting with its own
+// net (masked argmax); r_d(a) is the branch's final rewards[0].  With R_A, R_B the match's final rewards[0] at both tables:
+//   gain g_d(a) = sigma_p * (imp_of_difference(r_d(a) + R_other) - imp_of_difference(R_A + R_B)), sigma_p = +1 for players
+//   0/1 and -1 for 2/3: the change of the decider's team's match IMPs, the other table held at its result; an integer in
+//   [-48, 48].  regret_d = max over legal a of g_d(a) >= 0.  The played branch is the base game, so r_d(b_d) = R_T.
+constexpr int kCvStats = 4;  // {n, sum x, sum x^2, #(x > 0)}
+
+__device__ __forceinline__ int32_t call_value_gain(float r, float r_other, float base_imp, bool team1) {
+    const int32_t g = (int32_t)imp_of_difference(r + r_other) - (int32_t)base_imp;
+    return team1 ? g : -g;
+}
+
 __device__ __forceinline__ void history_set_bit(Env& e, uint32_t bit) {
     uint32_t w = bit >> 5, m = 1u << (bit & 31u);
 #pragma unroll

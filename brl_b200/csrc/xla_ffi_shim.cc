@@ -85,6 +85,7 @@
     X(brl_par_stats, "iiiiiiiix") \
     X(brl_system_stats, "iiiiix") \
     X(brl_system_stats_auctions, "iiiiix") \
+    X(brl_call_values, "iiiiiisoooooooooooo") \
     /* end */
 
 namespace {

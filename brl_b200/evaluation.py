@@ -497,6 +497,109 @@ def make_bidding_system_evaluate(eval_env, activation, model_type, num_eval_envs
     return system
 
 
+def call_values_bytes(n_envs: int, M: int, record_capacity: int = 0) -> int:
+    """device bytes of one chunk of make_call_values_evaluate for n_envs base envs and M nets (its pool not counted): the keys,
+    env_models, the two matches' scratch, cum_return, sums, status, both Table_infos, the int64 sums and the records"""
+    table_info = n_envs * (1 + 16 + 4 + 4 + 1 + 1)
+    sums = 8 * M * (ops._lib.SYS_CONTEXTS * (38 * 38 * 4 + 4) + 1)
+    records = record_capacity * (6 * 4 + 38 * 4) + 8 if record_capacity else 0
+    return (n_envs * (8 + 8 + 4) + ops.duplicate_match_scratch_bytes(n_envs, M) + 64 + 4 + 2 * table_info
+            + ops.call_values_scratch_bytes(n_envs, M) + sums + 4 + records)
+
+
+class _CallValueBuffers:
+    """Fixed-address buffers of one chunk shape (n base envs, M nets): the base match (brl_duplicate_match with its Table_infos)
+    and brl_call_values, so repeated calls relaunch both ops' cached graphs."""
+
+    def __init__(self, n: int, M: int, dev):
+        self.match = _MatchBuffers(n, M, 0, dev, with_models=True, with_tables=True)
+        self.scratch = torch.empty(ops.call_values_scratch_bytes(n, M), dtype=torch.uint8, device=dev)
+        self.gain = torch.empty((M,) + ops.CALL_GAIN_SHAPE, dtype=torch.int64, device=dev)
+        self.regret = torch.empty((M,) + ops.CALL_REGRET_SHAPE, dtype=torch.int64, device=dev)
+        self.mismatch = torch.empty(M, dtype=torch.int64, device=dev)
+        self.status = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.records = None
+
+
+def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):
+    """Counterfactual call values of M nets (DESIGN.md f16): `call_values(params_list, rng_key, opponent=None, records=False)`
+    plays the matches make_bidding_system_evaluate plays (net m in all four seats, or net m on players 0/1 against net k =
+    `opponent` on 2/3, every match on the same boards) and at every decision plays out every legal alternative call.  Returns
+    a dict of host int64 arrays: `gain_sums` [M, 75, 38, 38, 4] = {n, sum g, sum g^2, #(g > 0)} per (net, context, played,
+    alternative), `regret_sums` [M, 75, 4] = {decisions, sum regret, sum regret^2, #(regret > 0)} and `mismatch` [M]; with
+    `records=True` also this rank's decision records (dict of arrays env, table, player, net, context, played, r[., 38]; env =
+    global base env index m * num_eval_envs + board).
+    The M * num_eval_envs base envs are sharded over the ranks by global index (as the pair-match engine does), and each
+    rank plays its share in chunks of at most max_envs // 38 base envs, so that a chunk's 38 branch slots per env fit
+    `max_envs` branch rows.  Per chunk: one brl_duplicate_match (the base results) and one brl_call_values call; a chunk
+    holds call_values_bytes(chunk, M) device bytes.  The int64 sums are integers added in any order, with one all-reduce per
+    call, so they do not depend on the chunking or the rank count.  `tune`: BRL_F_TUNE_MLP_* bits pinning the forward."""
+    import numpy as np
+    forward_pass = make_forward_pass(activation=activation, model_type=model_type)
+    n, dev = num_eval_envs, eval_env.device
+    chunk = max(1, max_envs // ops.NUM_ACTIONS)
+    single_bf16 = forward_pass.precision == "tc-bf16"
+    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+    buffers = {}
+
+    def call_values(params_list, rng_key, opponent=None, records=False):
+        M = len(params_list)
+        if M < 1:
+            raise ValueError("make_call_values_evaluate: no nets given")
+        if opponent is not None and not 0 <= opponent < M:
+            raise ValueError(f"make_call_values_evaluate: opponent {opponent} is not a net of the {M} given")
+        rank, world = bdist.rank_world()
+        _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
+        board_keys = eval_env.make_keys(sub_key, n)
+        pairs = np.array([(m, m if opponent is None else opponent) for m in range(M)], dtype=np.int32)
+        total = torch.zeros(M * (int(np.prod(ops.CALL_GAIN_SHAPE)) + int(np.prod(ops.CALL_REGRET_SHAPE)) + 1), dtype=torch.int64,
+                            device=dev)
+        n_gain, n_regret = M * int(np.prod(ops.CALL_GAIN_SHAPE)), M * int(np.prod(ops.CALL_REGRET_SHAPE))
+        recs = []
+        lo, hi = bdist.shard_range(M * n, rank, world)
+        for c0 in range(lo, hi, chunk):
+            c1 = min(hi, c0 + chunk)
+            key = (c1 - c0, M)
+            if key not in buffers:
+                buffers[key] = _CallValueBuffers(c1 - c0, M, dev)
+            b = buffers[key]
+            for m, params in enumerate(params_list):
+                forward_pass.pack_into(params, b.match.pool[m, :blob_bytes])
+            g = np.arange(c0, c1)
+            b.match.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
+            b.match.env_models.copy_(torch.as_tensor(pairs[g // n], device=dev))
+            b.match.play(eval_env, single_bf16, tune)
+            if records and b.records is None:
+                b.records = ops.CallValueRecords(48 * (c1 - c0), dev)  # about twice a typical board's decisions
+            while True:
+                ops.call_values(b.match.keys, eval_env.table, b.match.pool, b.match.env_models, b.match.tables[0].rewards,
+                                b.match.tables[1].rewards, b.scratch, b.gain, b.regret, b.mismatch, b.status,
+                                records=b.records if records else None, env_offset=c0, single_bf16=single_bf16, tune=tune,
+                                illegal_penalty=eval_env.illegal_penalty, illegal_bonus=eval_env.illegal_bonus)
+                status = int(torch.maximum(b.status, b.match.status)[0])
+                if status != ops._lib.MATCH_RECORD_CAPACITY:
+                    break
+                b.records = ops.CallValueRecords(int(b.records.count[0]), dev)          # grow to the chunk's decisions
+            _check_match_status(status, "brl_call_values")
+            total[:n_gain] += b.gain.view(-1)
+            total[n_gain:n_gain + n_regret] += b.regret.view(-1)
+            total[n_gain + n_regret:] += b.mismatch
+            if records:
+                k = int(b.records.count[0])
+                recs.append({f: getattr(b.records, f)[:k].cpu().numpy() for f in ops.CALL_RECORD_FIELDS + ("r",)})
+        bdist.allreduce_sums(total)
+        host = total.cpu().numpy()
+        out = dict(gain_sums=host[:n_gain].reshape((M,) + ops.CALL_GAIN_SHAPE),
+                   regret_sums=host[n_gain:n_gain + n_regret].reshape((M,) + ops.CALL_REGRET_SHAPE),
+                   mismatch=host[n_gain + n_regret:])
+        if records:
+            out["records"] = {f: np.concatenate([r[f] for r in recs]) if recs else np.zeros((0,) + ((38,) if f == "r" else ()))
+                              for f in ops.CALL_RECORD_FIELDS + ("r",)}
+        return out
+
+    return call_values
+
+
 def make_device_pfsp_probe(eval_env, activation, model_type, num_eval_envs: int, max_envs: int = 1 << 20, *, tune: int = 0):
     """The PFSP probe of ppo.py:412-436 -- the learner against every model of a zoo.ModelZoo -- as one brl_duplicate_match
     call per chunk over the zoo's own pool (M = 1 + capacity nets, nothing copied per call).  The learner's parameters are

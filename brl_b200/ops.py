@@ -917,3 +917,73 @@ def system_stats_auctions(table: torch.Tensor, calls: torch.Tensor, offsets: tor
         raise _lib.BrlError("system_stats_auctions: a dealer is outside 0..3")
     _call("brl_system_stats_auctions", [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(board), _ptr(dealer), _ptr(hist)],
           _params(n, n_deals=table.shape[0]))
+
+
+# ---- counterfactual call values (DESIGN.md f16) ----------------------------------------------------------------------------
+CALL_GAIN_SHAPE = (_lib.SYS_CONTEXTS, NUM_ACTIONS, NUM_ACTIONS, 4)  # one net's gain sums: [context, played, alternative, stat]
+CALL_REGRET_SHAPE = (_lib.SYS_CONTEXTS, 4)                          # one net's regret sums: [context, stat]
+CALL_RECORD_FIELDS = ("env", "table", "player", "net", "context", "played")
+
+
+def call_values_scratch_bytes(n_envs: int, n_models: int) -> int:
+    return _size_query("brl_call_values_scratch_bytes", n_envs, n_models)
+
+
+class CallValueRecords:
+    """Record buffers of `call_values` for `capacity` decisions: int32 env, table, player, net, context, played [cap], f32
+    r[cap, 38] (NaN for an illegal call) and the int64 decision count[1] (also counted beyond the capacity)."""
+
+    def __init__(self, capacity: int, device):
+        self.capacity = int(capacity)
+        self.count = torch.zeros(1, dtype=torch.int64, device=device)
+        for f in CALL_RECORD_FIELDS:
+            setattr(self, f, torch.empty(self.capacity, dtype=torch.int32, device=device))
+        self.r = torch.empty((self.capacity, NUM_ACTIONS), dtype=torch.float32, device=device)
+
+    def ptrs(self):
+        return [_ptr(self.count)] + [_ptr(getattr(self, f)) for f in CALL_RECORD_FIELDS] + [_ptr(self.r)]
+
+
+def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env_models: torch.Tensor, rewards_a: torch.Tensor,
+                rewards_b: torch.Tensor, scratch: torch.Tensor, gain_sums: torch.Tensor, regret_sums: torch.Tensor,
+                mismatch: torch.Tensor, status: torch.Tensor, *, records: Optional[CallValueRecords] = None,
+                env_offset: int = 0, single_bf16: bool = False, tune: int = 0, illegal_penalty: float = -1.0,
+                illegal_bonus: float = 1.0) -> None:
+    """Replay the duplicate match `duplicate_match` plays for these keys, pool and env_models (int32 [n, 2] by team or
+    [n, 4] by player id) and, at every decision, play every legal alternative call out on that table with the nets' own
+    argmax (DESIGN.md f16).  rewards_a / rewards_b (f32 [n, 4]) are the final Table_info rewards of that match.  Writes
+    gain_sums int64 [M, 75, 38, 38, 4], regret_sums int64 [M, 75, 4], mismatch int64 [M], status int32[1] (_lib.MATCH_*) and,
+    with `records`, one record per decision (records' env = env_offset + i).  Nothing is read back to the host."""
+    n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
+    if keys.dtype != torch.int64 or keys.dim() != 1:
+        raise _lib.BrlError("call_values: keys must be int64 [n] (ops.make_keys)")
+    if pool.dim() != 2 or pool.dtype != torch.uint8 or pool.shape[1] != mlp_pool_stride() or M < 1:
+        raise _lib.BrlError("call_values: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    if env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4)):
+        raise _lib.BrlError("call_values: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    for name, t in (("rewards_a", rewards_a), ("rewards_b", rewards_b)):
+        if t.dtype != torch.float32 or tuple(t.shape) != (n, 4):
+            raise _lib.BrlError(f"call_values: {name} must be float32 [n, 4] (a Table_info's rewards)")
+    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
+        raise _lib.BrlError("call_values: the deal table must be u8 [n_deals, 48]")
+    if gain_sums.dtype != torch.int64 or tuple(gain_sums.shape) != (M,) + CALL_GAIN_SHAPE:
+        raise _lib.BrlError(f"call_values: gain_sums must be int64 [{M}, 75, 38, 38, 4]")
+    if regret_sums.dtype != torch.int64 or tuple(regret_sums.shape) != (M,) + CALL_REGRET_SHAPE:
+        raise _lib.BrlError(f"call_values: regret_sums must be int64 [{M}, 75, 4]")
+    if mismatch.dtype != torch.int64 or tuple(mismatch.shape) != (M,):
+        raise _lib.BrlError(f"call_values: mismatch must be int64 [{M}]")
+    if status.dtype != torch.int32 or status.numel() < 1:
+        raise _lib.BrlError("call_values: status must be int32 [1]")
+    if n and scratch.numel() < call_values_scratch_bytes(n, M):
+        raise _lib.BrlError("call_values: scratch too small (ops.call_values_scratch_bytes)")
+    if tune & F_SAMPLE:
+        raise _lib.BrlError("call_values: sampling is not supported (argmax only)")
+    if n and int(env_offset) < 0:
+        raise _lib.BrlError("call_values: env_offset must be >= 0")
+    flags = (F_MLP_BF16 if single_bf16 else 0) | (_lib.F_PLAYER_MODELS if env_models.shape[1] == 4 else 0) | tune
+    _call("brl_call_values", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(env_models), _ptr(rewards_a), _ptr(rewards_b),
+                              _ptr(scratch), _ptr(gain_sums), _ptr(regret_sums), _ptr(mismatch), _ptr(status)]
+          + (records.ptrs() if records is not None else [None] * 8),
+          _params(n, k_steps=M, n_deals=table.shape[0], flags=flags, env_offset=env_offset,
+                  seed=records.capacity if records is not None else 0, illegal_penalty=illegal_penalty,
+                  illegal_bonus=illegal_bonus))

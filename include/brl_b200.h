@@ -59,6 +59,8 @@
  *                         transition reward as IMPs against it, and a duplicate match's bidding against it (DESIGN.md f13)
  *   brl_system_stats / brl_system_stats_auctions   not in the reference: the hand strength and shape behind each call, by
  *                         net, context and call, counted in the match loop or over stored auctions (DESIGN.md f15)
+ *   brl_call_values       not in the reference: every legal alternative of every decision of a duplicate match played out,
+ *                         and the IMPs each would have changed, by net, context, played call and alternative (DESIGN.md f16)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -457,6 +459,38 @@ int32_t brl_system_stats(brl_stream_t, void **buffers, const void *opaque, size_
  * params: n_envs = n auctions. */
 int32_t brl_system_stats_auctions(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- counterfactual call values (not in the reference; DESIGN.md f16, restated by tests/call_values_ref.py) --------------
+ * The base match is the duplicate match brl_duplicate_match plays for the same keys, pool, env_models and flags; every
+ * decision is the masked argmax of the acting net.  A decision d is each step where env e is live at table T (A or B): the
+ * pre-step state S_d, the player p to act and its net m (brl_model_rows' rule), the context c of brl_system_stats, and the
+ * played call b_d.  For every call a legal in S_d the branch (d, a) starts from brl_step(S_d, a) (no auto-reset, no table
+ * switch) and plays that one table to its end, each player acting with its own net from env_models (masked argmax); r_d(a)
+ * is the branch's final rewards[0].  With R_A, R_B the base match's final rewards[0] at both tables:
+ *   gain   g_d(a) = sigma_p * (imp_of_difference(r_d(a) + R_other) - imp_of_difference(R_A + R_B)), sigma_p = +1 for players
+ *          0/1, -1 for 2/3: the change of the decider's team's match IMPs with the other table held at its result, in [-48, 48]
+ *   regret regret_d = max over legal a of g_d(a) >= 0 (a hindsight bound: the decider does not see the other hands)
+ * The played branch is the base game, so r_d(b_d) = R_T; the op counts the decisions where it is not (`mismatch`).
+ * Per base iteration the body forwards the base envs, writes 38 branch slots per env (an illegal call's or a finished env's
+ * slot is born finished), plays them out in a nested WHILE node (grouping by player, grouped forward, brl_step, control with a
+ * bound of 319 calls per auction), forms the gains, and only then steps the base envs with brl_duplicate_step.
+ * buffers: [0] in u64 keys[n]  [1] in deal_table  [2] in pool u8[M, brl_mlp_pool_stride()]
+ *          [3] in i32 env_models[n, 2] by team (or [n, 4] by player id with BRL_F_PLAYER_MODELS), 16-byte aligned
+ *          [4] in f32 rewards_a[n, 4], [5] in f32 rewards_b[n, 4]: the final Table_info rewards of brl_duplicate_match on the
+ *          same keys, nets and flags  [6] scratch (brl_call_values_scratch_bytes(n, M))
+ *          [7] out i64 gain_sums[M, 75, 38, 38, 4] = {n, sum g, sum g^2, #(g > 0)} per (net, context, played, alternative)
+ *          [8] out i64 regret_sums[M, 75, 4] = {decisions, sum regret, sum regret^2, #(regret > 0)}
+ *          [9] out i64 mismatch[M]: decisions with r_d(b_d) != R_T  [10] out i32 status[1] (BRL_MATCH_*)
+ *          [11] out i64 count[1] (the decisions, also beyond the capacity)  [12..17] out i32 env (env_offset + i), table (0 A,
+ *          1 B), player, net, context, played [cap]  [18] out f32 r[cap, 38] (NaN for an illegal call) -- the records, all
+ *          eight or none
+ * params: n_envs = n, k_steps = M, n_deals, env_offset (added to the records' env), seed = the record capacity cap,
+ *         illegal_penalty / illegal_bonus, flags BRL_F_PLAYER_MODELS | BRL_F_MLP_BF16 | BRL_F_TUNE_MLP_* (BRL_F_SAMPLE is an
+ *         error).  More decisions than cap set BRL_MATCH_RECORD_CAPACITY; the sums stay complete.  An empty batch is a
+ *         no-op.  The graph cache and capture rules are brl_duplicate_match's. */
+#define BRL_MATCH_RECORD_CAPACITY 3  /* brl_call_values: more decisions than record slots; every sum is still complete */
+int64_t brl_call_values_scratch_bytes(int64_t n_envs, int64_t n_models);
+int32_t brl_call_values(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -719,6 +753,7 @@ void brl_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque
 void brl_gather_reward_par_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_system_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_system_stats_auctions_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_call_values_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------
