@@ -17,7 +17,7 @@ from . import build as _build
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
             "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped",
             "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats",
-            "brl_system_stats", "brl_system_stats_auctions", "brl_call_values")
+            "brl_system_stats", "brl_system_stats_auctions", "brl_call_values", "brl_cv_grad", "brl_cv_eval")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",

@@ -5,7 +5,8 @@
 //                         the same loop with the step log (brl_eval_act_log) and the statistics (brl_eval_summary), or with
 //                         one env step per iteration and the actor's return
 //   brl_call_values       brl_duplicate_match's loop with, after each forward, every live env branched on every legal call and
-//                         the branches played out by a nested WHILE node (DESIGN.md f16)
+//                         the branches played out by a nested WHILE node (DESIGN.md f16); optionally each decision's
+//                         observation and gains as training examples (DESIGN.md f17)
 //
 //   init (brl_init) -> Table_info A / B (brl_state_fields) -> grouping (brl_model_rows) -> control
 //   WHILE (control said so) {
@@ -224,6 +225,32 @@ __global__ void __launch_bounds__(256) k_call_value_gains(const uint4* __restric
     o.context[k] = (int32_t)c;
     o.played[k] = b;
     for (int a = 0; a < kNumActions; ++a) o.r[k * kNumActions + a] = (legal >> a) & 1ull ? ri[a] : __int_as_float(0x7fc00000);
+}
+
+// Training examples of the records (DESIGN.md f17), in the graph only with buffers [19] / [20].  k_cv_mark saves the record
+// count before an iteration's k_call_value_gains; k_cv_examples then fills the slots that kernel took, [saved, min(count,
+// cap)), one warp per slot: the base env's bf16 observation row (what the forward of this iteration read: the branches
+// step their own buffers) and the gains of the record's r, NaN where r is (an illegal call).
+__global__ void k_cv_mark(const unsigned long long* __restrict__ count, unsigned long long* __restrict__ saved) { *saved = *count; }
+
+__global__ void __launch_bounds__(256) k_cv_examples(const uint4* __restrict__ obs, const float4* __restrict__ ra,
+                                                     const float4* __restrict__ rb, const CvOut o,
+                                                     const unsigned long long* __restrict__ saved, uint4* __restrict__ ex_obs,
+                                                     float* __restrict__ ex_gain) {
+    constexpr int kRow = BRL_OBS_DIM * 2 / 16;  // one bf16 row in 16-byte words
+    const int lane = threadIdx.x & 31;
+    const unsigned long long end = min(*o.count, (unsigned long long)o.cap);
+    const unsigned long long k = *saved + (((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (k >= end) return;
+    const int64_t i = (int64_t)o.env[k] - o.env_offset;
+    for (int w = lane; w < kRow; w += 32) ex_obs[k * kRow + w] = obs[i * kRow + w];
+    const float R_a = ra[i].x, R_b = rb[i].x, R_other = o.table[k] ? R_a : R_b;
+    const float base = imp_of_difference(R_a + R_b);
+    const bool team1 = o.player[k] < 2;
+    for (int a = lane; a < kNumActions; a += 32) {
+        const float r = o.r[k * kNumActions + a];
+        ex_gain[k * kNumActions + a] = isnan(r) ? r : (float)call_value_gain(r, R_other, base, team1);
+    }
 }
 
 // ---- the scratch ----------------------------------------------------------------------------------------------------------
@@ -683,6 +710,9 @@ struct CvPlan {
     const float4 *ra, *rb;
     float* r;
     CvOut o;
+    uint4* ex_obs;    // [19] training examples' bf16 obs[cap, 480] (NULL: none)
+    float* ex_gain;   // [20] their f32 gain[cap, 38]
+    unsigned long long* saved;  // the record count before the iteration's gains: a spare word of the base loop's ctl
 };
 
 // brl_step without auto-reset on the branch batch, then r += rewards[:, 0] (non-zero on a slot's last step only)
@@ -731,10 +761,14 @@ static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, c
         return rc;
     const int32_t* action = q.at<int32_t>(q.L.action);
     const uint8_t* a_done = static_cast<const uint8_t*>(q.info[0][0]);
+    if (c.ex_obs) k_cv_mark<<<1, 1, 0, s1>>>(c.o.count, c.saved);
     if (q.player_models)
         k_call_value_gains<4><<<blocks(q.n), 256, 0, s1>>>(state, done, q.env_models, action, a_done, c.ra, c.rb, c.r, c.o, q.n, q.M);
     else
         k_call_value_gains<2><<<blocks(q.n), 256, 0, s1>>>(state, done, q.env_models, action, a_done, c.ra, c.rb, c.r, c.o, q.n, q.M);
+    if (c.ex_obs)  // at most one record per base env and iteration: n warps
+        k_cv_examples<<<blocks(q.n * 32), 256, 0, s1>>>(static_cast<const uint4*>(q.obs), c.ra, c.rb, c.o, c.saved, c.ex_obs,
+                                                         c.ex_gain);
     if ((rc = launched(q.who, "gains")) || (rc = env_step(q, s1)) || (rc = model_rows(q, s1))) return rc;
     return cv_control(q, s1, loop, BRL_MATCH_MAX_STEPS);
 }
@@ -951,6 +985,12 @@ int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_
     if (given && (misaligned(b[11], 8) || misaligned(b[12], 4) || misaligned(b[13], 4) || misaligned(b[14], 4) ||
                   misaligned(b[15], 4) || misaligned(b[16], 4) || misaligned(b[17], 4) || misaligned(b[18], 4)))
         return fail(BRL_E_BUFFER, "brl_call_values: the record count must be 8-byte and the records 4-byte aligned");
+    const bool examples = b[19] != nullptr;
+    if (examples != (b[20] != nullptr))
+        return fail(BRL_E_BUFFER, "brl_call_values: give both training-example buffers [19] obs and [20] gain, or neither");
+    if (examples && !given) return fail(BRL_E_BUFFER, "brl_call_values: the training examples [19], [20] need the eight record buffers [11..18]");
+    if (examples && (misaligned(b[19], 16) || misaligned(b[20], 4)))
+        return fail(BRL_E_BUFFER, "brl_call_values: the example obs [19] must be 16-byte and gain [20] 4-byte aligned");
 
     CvPlan c{};
     c.q = base_plan("brl_call_values", 0, p, M, b[6]);
@@ -985,7 +1025,13 @@ int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_
         c.o.played = static_cast<int32_t*>(b[17]);
         c.o.r = static_cast<float*>(b[18]);
     }
-    return run_graph(c.q.who, (cudaStream_t)stream, p, b, 19, [&](cudaStream_t s0, cudaStream_t* side) {
+    if (examples) {
+        c.ex_obs = static_cast<uint4*>(b[19]);
+        c.ex_gain = static_cast<float*>(b[20]);
+        c.saved = reinterpret_cast<unsigned long long*>(c.q.at<unsigned char>(c.q.L.ctl) + 8);  // ctl holds one i32 in 16 bytes
+    }
+    // the cache key holds all 21 addresses: a graph with the example kernels and one without are two entries
+    return run_graph(c.q.who, (cudaStream_t)stream, p, b, 21, [&](cudaStream_t s0, cudaStream_t* side) {
         return emit_call_values(c, s0, side[1], side[2], side[3]);
     });
 }

@@ -86,6 +86,8 @@
     X(brl_system_stats, "iiiiix") \
     X(brl_system_stats_auctions, "iiiiix") \
     X(brl_call_values, "iiiiiisoooooooooooo") \
+    X(brl_cv_grad, "iisioos") \
+    X(brl_cv_eval, "iisios") \
     /* end */
 
 namespace {

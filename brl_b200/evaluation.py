@@ -528,7 +528,11 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
     a dict of host int64 arrays: `gain_sums` [M, 75, 38, 38, 4] = {n, sum g, sum g^2, #(g > 0)} per (net, context, played,
     alternative), `regret_sums` [M, 75, 4] = {decisions, sum regret, sum regret^2, #(regret > 0)} and `mismatch` [M]; with
     `records=True` also this rank's decision records (dict of arrays env, table, player, net, context, played, r[., 38]; env =
-    global base env index m * num_eval_envs + board).
+    global base env index m * num_eval_envs + board).  `records="train"` also returns this rank's training examples
+    (DESIGN.md f17) as device tensors, `examples` = dict(obs bf16 [k, 480], gain f32 [k, 38] (NaN: illegal), net int32 [k]),
+    row k belonging to record k; the records and examples are then ordered by env, table and play order, so that a seeded
+    run repeats them row for row.  `matches`: the (net on players 0/1, net on players 2/3) pairs to play instead, match j on
+    global base envs j * num_eval_envs + board (e.g. [(0, 1)]: only net 0 against net 1).
     The M * num_eval_envs base envs are sharded over the ranks by global index (as the pair-match engine does), and each
     rank plays its share in chunks of at most max_envs // 38 base envs, so that a chunk's 38 branch slots per env fit
     `max_envs` branch rows.  Per chunk: one brl_duplicate_match (the base results) and one brl_call_values call; a chunk
@@ -542,21 +546,30 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
     blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
     buffers = {}
 
-    def call_values(params_list, rng_key, opponent=None, records=False):
+    def call_values(params_list, rng_key, opponent=None, records=False, matches=None):
         M = len(params_list)
         if M < 1:
             raise ValueError("make_call_values_evaluate: no nets given")
         if opponent is not None and not 0 <= opponent < M:
             raise ValueError(f"make_call_values_evaluate: opponent {opponent} is not a net of the {M} given")
+        if matches is not None and (opponent is not None or not matches or
+                                    any(len(mt) != 2 or not all(0 <= x < M for x in mt) for mt in matches)):
+            raise ValueError(f"make_call_values_evaluate: matches must be (net on players 0/1, net on 2/3) pairs of the {M} "
+                             "nets, without `opponent`")
+        if records not in (False, True, "train"):
+            raise ValueError(f"make_call_values_evaluate: records must be False, True or 'train', got {records!r}")
         rank, world = bdist.rank_world()
         _, sub_key = brandom.split(rng_key)                                                # as duplicate_evaluate
         board_keys = eval_env.make_keys(sub_key, n)
-        pairs = np.array([(m, m if opponent is None else opponent) for m in range(M)], dtype=np.int32)
+        train = records == "train"
+        examples = []
+        pairs = np.array(matches if matches is not None else [(m, m if opponent is None else opponent) for m in range(M)],
+                         dtype=np.int32).reshape(-1, 2)
         total = torch.zeros(M * (int(np.prod(ops.CALL_GAIN_SHAPE)) + int(np.prod(ops.CALL_REGRET_SHAPE)) + 1), dtype=torch.int64,
                             device=dev)
         n_gain, n_regret = M * int(np.prod(ops.CALL_GAIN_SHAPE)), M * int(np.prod(ops.CALL_REGRET_SHAPE))
         recs = []
-        lo, hi = bdist.shard_range(M * n, rank, world)
+        lo, hi = bdist.shard_range(len(pairs) * n, rank, world)
         for c0 in range(lo, hi, chunk):
             c1 = min(hi, c0 + chunk)
             key = (c1 - c0, M)
@@ -569,8 +582,8 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
             b.match.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
             b.match.env_models.copy_(torch.as_tensor(pairs[g // n], device=dev))
             b.match.play(eval_env, single_bf16, tune)
-            if records and b.records is None:
-                b.records = ops.CallValueRecords(48 * (c1 - c0), dev)  # about twice a typical board's decisions
+            if records and (b.records is None or b.records.train != train):
+                b.records = ops.CallValueRecords(48 * (c1 - c0), dev, train)  # about twice a typical board's decisions
             while True:
                 ops.call_values(b.match.keys, eval_env.table, b.match.pool, b.match.env_models, b.match.tables[0].rewards,
                                 b.match.tables[1].rewards, b.scratch, b.gain, b.regret, b.mismatch, b.status,
@@ -579,14 +592,23 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
                 status = int(torch.maximum(b.status, b.match.status)[0])
                 if status != ops._lib.MATCH_RECORD_CAPACITY:
                     break
-                b.records = ops.CallValueRecords(int(b.records.count[0]), dev)          # grow to the chunk's decisions
+                b.records = ops.CallValueRecords(int(b.records.count[0]), dev, train)  # grow to the chunk's decisions
             _check_match_status(status, "brl_call_values")
             total[:n_gain] += b.gain.view(-1)
             total[n_gain:n_gain + n_regret] += b.regret.view(-1)
             total[n_gain + n_regret:] += b.mismatch
             if records:
                 k = int(b.records.count[0])
-                recs.append({f: getattr(b.records, f)[:k].cpu().numpy() for f in ops.CALL_RECORD_FIELDS + ("r",)})
+                if not train:
+                    recs.append({f: getattr(b.records, f)[:k].cpu().numpy() for f in ops.CALL_RECORD_FIELDS + ("r",)})
+                else:
+                    # the slots follow the gains kernel's atomics; an (env, table)'s slots rise in play order, so a stable
+                    # sort by (env, table) gives an order that a seeded run repeats.  Gathered copies: the buffers are
+                    # reused by the next chunk and the next call.
+                    r = b.records
+                    order = torch.sort(r.env[:k].long() * 2 + r.table[:k], stable=True).indices
+                    recs.append({f: getattr(r, f)[:k][order].cpu().numpy() for f in ops.CALL_RECORD_FIELDS + ("r",)})
+                    examples.append((r.obs[:k][order], r.gain[:k][order], r.net[:k][order]))
         bdist.allreduce_sums(total)
         host = total.cpu().numpy()
         out = dict(gain_sums=host[:n_gain].reshape((M,) + ops.CALL_GAIN_SHAPE),
@@ -595,6 +617,11 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
         if records:
             out["records"] = {f: np.concatenate([r[f] for r in recs]) if recs else np.zeros((0,) + ((38,) if f == "r" else ()))
                               for f in ops.CALL_RECORD_FIELDS + ("r",)}
+        if train:
+            out["examples"] = dict(
+                obs=torch.cat([e[0] for e in examples]) if examples else torch.zeros((0, ops.OBS_DIM), dtype=torch.bfloat16, device=dev),
+                gain=torch.cat([e[1] for e in examples]) if examples else torch.zeros((0, 38), dtype=torch.float32, device=dev),
+                net=torch.cat([e[2] for e in examples]) if examples else torch.zeros(0, dtype=torch.int32, device=dev))
         return out
 
     return call_values

@@ -602,6 +602,42 @@ def sl_eval(obs, blob, scratch, mask, label, stats, acc, *, ent_coef=0.0) -> Non
     _call("brl_sl_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(stats), _ptr(acc)], p)
 
 
+CV_WIDE_FORWARD, CV_NARROW_BACKWARD = 1 << 16, 1 << 17  # brl_cv_grad's tile-width experiment bits (BRL_CV_*)
+
+
+def _cv_params(name, obs, gain, scratch, blob, ent_coef, tiles=0):
+    L = _lib.load()
+    B = int(gain.shape[0])
+    if obs.dtype == torch.bool:
+        obs = obs.view(torch.uint8)
+    if gain.dtype != torch.float32 or tuple(gain.shape) != (B, NUM_ACTIONS):
+        raise _lib.BrlError(f"{name}: gain must be float32 [B, 38] (NaN for an illegal call)")
+    if tuple(obs.shape) != (B, OBS_DIM):
+        raise _lib.BrlError(f"{name}: obs must be [B, 480] with B = gain.shape[0]")
+    if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
+        raise _lib.BrlError(f"{name}: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
+    if tiles & ~(CV_WIDE_FORWARD | CV_NARROW_BACKWARD):
+        raise _lib.BrlError(f"{name}: tiles takes CV_WIDE_FORWARD / CV_NARROW_BACKWARD only")
+    return obs, _lib.BrlSlParams(B, float(ent_coef), obs_flag(obs.dtype) | tiles)
+
+
+def cv_grad(obs, blob, scratch, gain, grads, stats, acc, *, ent_coef=0.0, tiles=0) -> None:
+    """One minibatch of the call-value policy-improvement loss (DESIGN.md f17) through the MLP on tcgen05: gain f32[B, 38]
+    (IMPs, NaN = illegal), loss = -mean(sum_a pi_a g_a) / 24 - ent_coef * mean entropy -> flat fp32 gradients, stats[8]
+    (include/brl_b200.h brl_cv_grad) and acc[14] = sum of squares of the gradient (sl_acc's buffer).  `tiles`: the
+    CV_WIDE_FORWARD / CV_NARROW_BACKWARD experiment bits (0: the measured tile widths)."""
+    obs, p = _cv_params("cv_grad", obs, gain, scratch, blob, ent_coef, tiles)
+    if grads.dtype != torch.float32 or grads.numel() != _lib.load().brl_mlp_num_params():
+        raise _lib.BrlError("cv_grad: grads must be the flat fp32 gradient buffer")
+    _call("brl_cv_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(gain), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+
+
+def cv_eval(obs, blob, scratch, gain, stats, acc, *, ent_coef=0.0, tiles=0) -> None:
+    """cv_grad's statistics without the backward (bit-equal to cv_grad's on the same inputs)."""
+    obs, p = _cv_params("cv_eval", obs, gain, scratch, blob, ent_coef, tiles)
+    _call("brl_cv_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(gain), _ptr(stats), _ptr(acc)], p)
+
+
 def gather_rows(src: torch.Tensor, index: torch.Tensor, dst: torch.Tensor) -> None:
     """dst[b] = src[index[b]] over the leading axis (minibatch take, src/update.py:194-199)."""
     row_bytes = src[0].numel() * src.element_size()
@@ -931,17 +967,23 @@ def call_values_scratch_bytes(n_envs: int, n_models: int) -> int:
 
 class CallValueRecords:
     """Record buffers of `call_values` for `capacity` decisions: int32 env, table, player, net, context, played [cap], f32
-    r[cap, 38] (NaN for an illegal call) and the int64 decision count[1] (also counted beyond the capacity)."""
+    r[cap, 38] (NaN for an illegal call) and the int64 decision count[1] (also counted beyond the capacity).  With `train`
+    also the training examples of DESIGN.md f17: bf16 obs[cap, 480] (the observation the acting net read) and f32
+    gain[cap, 38] (g_d(a) in IMPs, NaN where the call is illegal), row k belonging to record k."""
 
-    def __init__(self, capacity: int, device):
+    def __init__(self, capacity: int, device, train: bool = False):
         self.capacity = int(capacity)
         self.count = torch.zeros(1, dtype=torch.int64, device=device)
         for f in CALL_RECORD_FIELDS:
             setattr(self, f, torch.empty(self.capacity, dtype=torch.int32, device=device))
         self.r = torch.empty((self.capacity, NUM_ACTIONS), dtype=torch.float32, device=device)
+        self.train = bool(train)
+        self.obs = torch.empty((self.capacity, OBS_DIM), dtype=torch.bfloat16, device=device) if train else None
+        self.gain = torch.empty((self.capacity, NUM_ACTIONS), dtype=torch.float32, device=device) if train else None
 
     def ptrs(self):
-        return [_ptr(self.count)] + [_ptr(getattr(self, f)) for f in CALL_RECORD_FIELDS] + [_ptr(self.r)]
+        return ([_ptr(self.count)] + [_ptr(getattr(self, f)) for f in CALL_RECORD_FIELDS] + [_ptr(self.r)]
+                + [_ptr(self.obs), _ptr(self.gain)])
 
 
 def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env_models: torch.Tensor, rewards_a: torch.Tensor,
@@ -953,7 +995,8 @@ def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env
     [n, 4] by player id) and, at every decision, play every legal alternative call out on that table with the nets' own
     argmax (DESIGN.md f16).  rewards_a / rewards_b (f32 [n, 4]) are the final Table_info rewards of that match.  Writes
     gain_sums int64 [M, 75, 38, 38, 4], regret_sums int64 [M, 75, 4], mismatch int64 [M], status int32[1] (_lib.MATCH_*) and,
-    with `records`, one record per decision (records' env = env_offset + i).  Nothing is read back to the host."""
+    with `records`, one record per decision (records' env = env_offset + i), and with records made with `train=True` each
+    record's training example (obs, gain; DESIGN.md f17).  Nothing is read back to the host."""
     n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
     if keys.dtype != torch.int64 or keys.dim() != 1:
         raise _lib.BrlError("call_values: keys must be int64 [n] (ops.make_keys)")
@@ -983,7 +1026,7 @@ def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env
     flags = (F_MLP_BF16 if single_bf16 else 0) | (_lib.F_PLAYER_MODELS if env_models.shape[1] == 4 else 0) | tune
     _call("brl_call_values", [_ptr(keys), _ptr(table), _ptr(pool), _ptr(env_models), _ptr(rewards_a), _ptr(rewards_b),
                               _ptr(scratch), _ptr(gain_sums), _ptr(regret_sums), _ptr(mismatch), _ptr(status)]
-          + (records.ptrs() if records is not None else [None] * 8),
+          + (records.ptrs() if records is not None else [None] * 10),
           _params(n, k_steps=M, n_deals=table.shape[0], flags=flags, env_offset=env_offset,
                   seed=records.capacity if records is not None else 0, illegal_penalty=illegal_penalty,
                   illegal_bonus=illegal_bonus))

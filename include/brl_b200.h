@@ -60,7 +60,10 @@
  *   brl_system_stats / brl_system_stats_auctions   not in the reference: the hand strength and shape behind each call, by
  *                         net, context and call, counted in the match loop or over stored auctions (DESIGN.md f15)
  *   brl_call_values       not in the reference: every legal alternative of every decision of a duplicate match played out,
- *                         and the IMPs each would have changed, by net, context, played call and alternative (DESIGN.md f16)
+ *                         and the IMPs each would have changed, by net, context, played call and alternative (DESIGN.md f16);
+ *                         optionally each decision's observation and gains as training examples (DESIGN.md f17)
+ *   brl_cv_grad / brl_cv_eval   not in the reference: the all-actions policy-gradient loss head on those examples, on the
+ *                         tensor-core forward / backward of brl_sl_grad (DESIGN.md f17)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -483,6 +486,10 @@ int32_t brl_system_stats_auctions(brl_stream_t, void **buffers, const void *opaq
  *          [11] out i64 count[1] (the decisions, also beyond the capacity)  [12..17] out i32 env (env_offset + i), table (0 A,
  *          1 B), player, net, context, played [cap]  [18] out f32 r[cap, 38] (NaN for an illegal call) -- the records, all
  *          eight or none
+ *          [19] out bf16 obs[cap, 480]: the observation row the acting net's forward read at record k's decision
+ *          [20] out f32 gain[cap, 38]: record k's g_d(a), NaN exactly where the call is illegal -- the training examples of
+ *          DESIGN.md f17 (row k belongs to record k), both or neither, and only with the records; obs 16-byte aligned.
+ *          Without them the graph is the one without the feature; through the XLA target they are NULL.
  * params: n_envs = n, k_steps = M, n_deals, env_offset (added to the records' env), seed = the record capacity cap,
  *         illegal_penalty / illegal_bonus, flags BRL_F_PLAYER_MODELS | BRL_F_MLP_BF16 | BRL_F_TUNE_MLP_* (BRL_F_SAMPLE is an
  *         error).  More decisions than cap set BRL_MATCH_RECORD_CAPACITY; the sums stay complete.  An empty batch is a
@@ -669,6 +676,29 @@ int32_t brl_sl_grad(brl_stream_t, void **buffers, const void *opaque, size_t opa
  * buffers: [0] in obs  [1] in blob  [2] scratch  [3] in u8 mask[B,38]  [4] in i32 label[B]  [5] out f32 stats[8]  [6] scratch f64[16] */
 int32_t brl_sl_eval(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- call-value policy improvement (not in the reference; DESIGN.md f17, restated by tests/cvi_ref.py) -----------------
+ * An all-actions policy-gradient step on brl_call_values' training examples: sample b has the gains g[b, a] of every call
+ * (NaN: illegal; the legal set is isfinite(g)).  pi = softmax of the logits over the legal calls, gbar = sum_a pi_a g_a,
+ * J_b = gbar / 24 (the IMP scale of reward_mode "par_imp"), H_b = entropy of pi.
+ *   loss = -mean_b J_b - ent_coef * mean_b H_b
+ *   d loss / d l_j = -pi_j (g_j - gbar) / (24 B) + ent_coef * pi_j (log pi_j + H_b) / B for legal j, 0 otherwise; the value
+ *   head gets no gradient.  A sample without a legal call contributes 0 to everything and 1 to stat 6.
+ * Follow with brl_mlp_adam_step.  opaque = BrlSlParams (batch, ent_coef, flags BRL_F_OBS_U8 / BRL_F_OBS_BF16, and the
+ * experiment bits BRL_CV_WIDE_FORWARD / BRL_CV_NARROW_BACKWARD: the other tile width of the fused forward (128x128) /
+ * backward (128x64) launch, as BrlPpoParams.reserved bits 4 / 16; 0 = the measured defaults).
+ * buffers: [0] in obs[B,480]  [1] in blob (brl_mlp_pack_train)  [2] scratch[brl_mlp_train_scratch_bytes(B)]
+ *          [3] in f32 gain[B,38]  [4] out f32 grads[brl_mlp_num_params()]
+ *          [5] out f32 stats[8] = {total loss, mean gbar (IMPs), mean g of the argmax-logit legal call (lowest index on
+ *              ties), mean (max_a g_a - that gain), mean entropy, share of samples whose argmax-logit call has the maximal g,
+ *              mean unmasked-softmax mass on illegal calls, 0}
+ *          [6] scratch f64[16] (BRL_SL_ACC_BYTES, 16-byte aligned; element 14 = sum of squares of grads) */
+#define BRL_CV_WIDE_FORWARD    (1 << 16)
+#define BRL_CV_NARROW_BACKWARD (1 << 17)
+int32_t brl_cv_grad(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+/* brl_cv_grad's forward and statistics without the backward (the same stats, bit for bit).
+ * buffers: [0] in obs  [1] in blob  [2] scratch  [3] in f32 gain[B,38]  [4] out f32 stats[8]  [5] scratch f64[16] */
+int32_t brl_cv_eval(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- full evaluation statistics (src/evaluation.py:207-1032) ---------------------------------- */
 #define BRL_F_EVAL_INDICATOR_BIDS 0x0400 /* non-duplicate `evaluate`: bid histogram is .set(1), not += 1 (src/evaluation.py:345-354) */
 #define BRL_EVAL_ACC_COLS 76    /* per-env log row: ill[2] steps[2] passes[2] actor_bid[35] opp_bid[35] (team 1 first) */
@@ -754,6 +784,8 @@ void brl_gather_reward_par_xla(brl_stream_t, void **buffers, const char *opaque,
 void brl_system_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_system_stats_auctions_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_call_values_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_cv_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_cv_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------

@@ -8,8 +8,9 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the counterfactual call values: no kernel is renamed, and k_cv_control, k_branch_calls and
-k_call_value_gains (per team <2> and per player <4>) are new.  Replace both tables for another change."""
+RENAMES and ADDED record call-value policy improvement (DESIGN.md f17): no kernel is renamed, and the loss head k_cv_loss
+and the two training-example kernels of brl_call_values, k_cv_mark and k_cv_examples, are new.  Replace both tables for
+another change."""
 import argparse
 import os
 import re
@@ -18,7 +19,7 @@ import sys
 from collections import OrderedDict
 
 RENAMES = []  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-ADDED = [r"^brl::k_cv_control$", r"^brl::k_branch_calls<\(int\)[24]>$", r"^brl::k_call_value_gains<\(int\)[24]>$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
+ADDED = [r"^brl::k_cv_loss$", r"^brl::k_cv_mark$", r"^brl::k_cv_examples$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):
