@@ -4,10 +4,7 @@
 //   brl_cv_grad      value_and_grad of the loss below for one minibatch: launch_train_minibatch with k_cv_loss as the head
 //   brl_cv_eval      the same statistics without the backward
 // The optimizer step is brl_mlp_adam_step (cvi.py: eps 1e-5 and global clipping, as ppo.train builds it).
-#include <cuda_bf16.h>
-#include <math.h>
-
-#include "common.h"
+#include "loss_head.cuh"
 
 namespace brl {
 
@@ -15,7 +12,7 @@ namespace brl {
 // The per-sample statistics are summed as 2^-30 fixed point in int64 (exact, so independent of the block order: two calls
 // on the same inputs, and brl_cv_grad / brl_cv_eval, give bit-equal stats); |x| <= 96 per sample and B <= 2^24 stay
 // below 2^61.
-enum { kCvAccGbar = 0, kCvAccEnt, kCvAccGarg, kCvAccRegret, kCvAccHit, kCvAccIllegal, kCvAccN, kCvAccSumsq = 14, kCvAccTicket = 15 };
+enum { kCvAccGbar = 0, kCvAccEnt, kCvAccGarg, kCvAccRegret, kCvAccHit, kCvAccIllegal, kCvAccN, kCvAccTicket = 15 };  // 14: |grads|^2 (sl_params_minibatch)
 constexpr double kCvFix = 1073741824.0;  // 2^30
 constexpr float kCvImpScale = 24.0f;     // J_b = gbar / 24: the IMP scale of reward_mode "par_imp"
 
@@ -32,21 +29,6 @@ struct CvLossArgs {
     float ent_coef;
 };
 
-__device__ __forceinline__ float cv_warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float cv_warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-__device__ __forceinline__ void cv_split_store(const CvLossArgs& a, int64_t idx, float v) {
-    const __nv_bfloat16 h = __float2bfloat16_rn(v), l = __float2bfloat16_rn(v - __bfloat162float(h));
-    a.dz_hi[idx] = *reinterpret_cast<const unsigned short*>(&h);
-    a.dz_lo[idx] = *reinterpret_cast<const unsigned short*>(&l);
-}
 __device__ __forceinline__ long long cv_fix(float v) { return __double2ll_rn((double)v * kCvFix); }
 
 // stats = {total loss, mean gbar, mean g(argmax), mean regret of the argmax, entropy, argmax-is-best share, illegal mass, 0};
@@ -66,7 +48,7 @@ __device__ __forceinline__ void cv_finalize(const CvLossArgs& a) {
     a.stats[7] = 0.0f;
 }
 
-// One warp per sample, lane owns calls lane and lane + 32 (k_sl_loss's layout).  Legal = isfinite(gain).
+// One warp per sample, lane owns calls lane and lane + 32 (loss_head.cuh).  Legal = isfinite(gain).
 //   pi = softmax over the legal calls, gbar = sum pi_a g_a, H = entropy of pi
 //   loss = -mean(gbar) / 24 - ent_coef * mean(H)
 //   d loss / d l_j = -pi_j (g_j - gbar) / (24 B) + ent_coef * pi_j (log pi_j + H) / B (legal j), 0 otherwise; d / d value = 0
@@ -92,11 +74,11 @@ __global__ void __launch_bounds__(128) k_cv_loss(const CvLossArgs a) {
         }
         const bool any = __any_sync(0xffffffffu, legal[0] || legal[1]);
         // unmasked softmax: the illegal mass
-        const float mx = cv_warp_max(fmaxf(l[0], l[1]));
-        const float lse = mx + logf(cv_warp_sum((in[0] ? expf(l[0] - mx) : 0.0f) + (in[1] ? expf(l[1] - mx) : 0.0f)));
+        const float mx = warp_max(fmaxf(l[0], l[1]));
+        const float lse = mx + logf(warp_sum((in[0] ? expf(l[0] - mx) : 0.0f) + (in[1] ? expf(l[1] - mx) : 0.0f)));
 #pragma unroll
         for (int k = 0; k < 2; ++k) q[k] = in[k] ? expf(l[k] - lse) : 0.0f;
-        const float ill = cv_warp_sum((in[0] && !legal[0] ? q[0] : 0.0f) + (in[1] && !legal[1] ? q[1] : 0.0f));
+        const float ill = warp_sum((in[0] && !legal[0] ? q[0] : 0.0f) + (in[1] && !legal[1] ? q[1] : 0.0f));
         if (!any) {
             if (a.dlogits) {
 #pragma unroll
@@ -104,25 +86,19 @@ __global__ void __launch_bounds__(128) k_cv_loss(const CvLossArgs a) {
                     const int j = lane + 32 * k;
                     if (!in[k]) continue;
                     a.dlogits[b * BRL_NUM_ACTIONS + j] = 0.0f;
-                    cv_split_store(a, b * 64 + j, 0.0f);
+                    store_dz(a.dz_hi, a.dz_lo, b * 64 + j, 0.0f);
                 }
-                if (lane >= 6) cv_split_store(a, b * 64 + 32 + lane, 0.0f);
+                if (lane >= 6) store_dz(a.dz_hi, a.dz_lo, b * 64 + 32 + lane, 0.0f);
                 if (lane == 0) a.dvalue[b] = 0.0f;
             }
             if (lane == 0) s[kCvAccIllegal] += cv_fix(ill);
             continue;
         }
         // softmax over the legal calls
-        const float mxl = cv_warp_max(fmaxf(legal[0] ? l[0] : -INFINITY, legal[1] ? l[1] : -INFINITY));
-        const float lsel = mxl + logf(cv_warp_sum((legal[0] ? expf(l[0] - mxl) : 0.0f) + (legal[1] ? expf(l[1] - mxl) : 0.0f)));
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-            logp[k] = legal[k] ? l[k] - lsel : -INFINITY;
-            p[k] = legal[k] ? expf(logp[k]) : 0.0f;
-        }
-        const float ent = -cv_warp_sum((legal[0] && p[0] > 0.0f ? p[0] * logp[0] : 0.0f) + (legal[1] && p[1] > 0.0f ? p[1] * logp[1] : 0.0f));
-        const float gbar = cv_warp_sum((legal[0] ? p[0] * g[0] : 0.0f) + (legal[1] ? p[1] * g[1] : 0.0f));
-        const float gmax = cv_warp_max(fmaxf(legal[0] ? g[0] : -INFINITY, legal[1] ? g[1] : -INFINITY));
+        softmax_sel(l, legal, p, logp);
+        const float ent = -warp_sum((legal[0] && p[0] > 0.0f ? p[0] * logp[0] : 0.0f) + (legal[1] && p[1] > 0.0f ? p[1] * logp[1] : 0.0f));
+        const float gbar = warp_sum((legal[0] ? p[0] * g[0] : 0.0f) + (legal[1] ? p[1] * g[1] : 0.0f));
+        const float gmax = warp_max(fmaxf(legal[0] ? g[0] : -INFINITY, legal[1] ? g[1] : -INFINITY));
         // argmax of the legal logits, lowest index on ties
         float best = legal[0] ? l[0] : -INFINITY, bg = g[0];
         int arg = legal[0] ? lane : 64;
@@ -144,9 +120,9 @@ __global__ void __launch_bounds__(128) k_cv_loss(const CvLossArgs a) {
                     if (p[k] > 0.0f) d += a.ent_coef * invB * p[k] * (logp[k] + ent);
                 }
                 a.dlogits[b * BRL_NUM_ACTIONS + j] = d;
-                cv_split_store(a, b * 64 + j, d);
+                store_dz(a.dz_hi, a.dz_lo, b * 64 + j, d);
             }
-            if (lane >= 6) cv_split_store(a, b * 64 + 32 + lane, 0.0f);  // the value column (38) and the padding 39..63
+            if (lane >= 6) store_dz(a.dz_hi, a.dz_lo, b * 64 + 32 + lane, 0.0f);  // the value column (38) and the padding 39..63
         }
         if (lane == 0) {
             if (a.dlogits) a.dvalue[b] = 0.0f;
@@ -158,45 +134,16 @@ __global__ void __launch_bounds__(128) k_cv_loss(const CvLossArgs a) {
             s[kCvAccIllegal] += cv_fix(ill);
         }
     }
-    // block sums, then the last block to arrive forms the statistics (k_sl_loss's ticket)
-    __shared__ long long part[4][kCvAccN];
-    __shared__ bool last_block;
-    const int w = threadIdx.x >> 5;
-    if (lane == 0)
-        for (int k = 0; k < kCvAccN; ++k) part[w][k] = s[k];
-    __syncthreads();
-    if (threadIdx.x < kCvAccN) {
-        const int k = threadIdx.x;
-        atomicAdd(reinterpret_cast<unsigned long long*>(&a.acc[k]),
-                  (unsigned long long)(part[0][k] + part[1][k] + part[2][k] + part[3][k]));
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const unsigned long long t = atomicAdd(reinterpret_cast<unsigned long long*>(&a.acc[kCvAccTicket]), 1ull);
-        last_block = t == (unsigned long long)gridDim.x - 1ull;
-    }
-    __syncthreads();
-    if (last_block && threadIdx.x == 0) {
-        __threadfence();
-        cv_finalize(a);
-    }
+    if (head_block_sums(s, a.acc, kCvAccTicket)) cv_finalize(a);
 }
 
-struct CvHead {
-    const float* gain;
-    float* stats;
-    double* acc;
-    int64_t B;
-    float ent_coef;
-    bool backward;
-};
-
+// brl_cv_grad: [0] obs [1] blob [2] scratch [3] gain [4] grads [5] stats [6] acc
+// brl_cv_eval: [0] obs [1] blob [2] scratch [3] gain [4] stats [5] acc
 static int32_t cv_loss_head(cudaStream_t s, const TrainHeadIO& io, const void* ctx) {
-    const CvHead& h = *static_cast<const CvHead*>(ctx);
+    const SlHeadCtx& h = *static_cast<const SlHeadCtx*>(ctx);
     CvLossArgs a{};
     a.logits = io.logits;
-    a.gain = h.gain;
+    a.gain = static_cast<const float*>(h.in[0]);
     if (h.backward) {
         a.dlogits = io.dlogits;
         a.dvalue = io.dvalue;
@@ -207,50 +154,12 @@ static int32_t cv_loss_head(cudaStream_t s, const TrainHeadIO& io, const void* c
     a.acc = h.acc;
     a.B = h.B;
     a.ent_coef = h.ent_coef;
-    unsigned grid = (unsigned)((h.B + 3) / 4);
-    if (grid > 148u * 8u) grid = 148u * 8u;
-    launch_pdl(k_cv_loss, dim3(grid), dim3(128), 0, s, a);
+    launch_pdl(k_cv_loss, dim3(head_grid(h.B)), dim3(128), 0, s, a);
     return check_launch(h.backward ? "brl_cv_grad (loss head)" : "brl_cv_eval (loss head)");
 }
 
-// brl_cv_grad: [0] obs [1] blob [2] scratch [3] gain [4] grads [5] stats [6] acc
-// brl_cv_eval: [0] obs [1] blob [2] scratch [3] gain [4] stats [5] acc
-static int32_t cv_minibatch(const char* what, cudaStream_t s, void** b, const void* opaque, size_t len, bool backward) {
-    if (opaque == nullptr || len != sizeof(BrlSlParams))
-        return fail(BRL_E_OPAQUE, "%s: opaque must be one BrlSlParams (%zu bytes), got %zu", what, sizeof(BrlSlParams), len);
-    const BrlSlParams* p = static_cast<const BrlSlParams*>(opaque);
-    if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "%s: batch must be in [0, 2^24]", what);
-    if (p->batch == 0) return BRL_OK;
-    static const char* grad_names[] = {"obs", "blob", "scratch", "gain", "grads", "stats", "acc"};
-    static const char* eval_names[] = {"obs", "blob", "scratch", "gain", "stats", "acc"};
-    // obs, blob, scratch, grads and acc 16-byte aligned
-    const int32_t rc = backward ? check_buffers(what, b, grad_names, 7, 0, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 4 | 1u << 6)
-                                : check_buffers(what, b, eval_names, 6, 0, 1u << 0 | 1u << 1 | 1u << 2 | 1u << 5);
-    if (rc != BRL_OK) return rc;
-    if ((reinterpret_cast<uintptr_t>(b[3]) & 3u) != 0) return fail(BRL_E_BUFFER, "%s: gain is not 4-byte aligned", what);
-    CvHead head{};
-    head.gain = static_cast<const float*>(b[3]);
-    head.stats = static_cast<float*>(b[backward ? 5 : 4]);
-    head.acc = static_cast<double*>(b[backward ? 6 : 5]);
-    head.B = p->batch;
-    head.ent_coef = p->ent_coef;
-    head.backward = backward;
-    TrainMinibatch t{};
-    t.obs = b[0];
-    t.obs_flags = p->flags & (BRL_F_OBS_U8 | BRL_F_OBS_BF16);  // same bits as BRL_PPO_OBS_U8 / BRL_PPO_OBS_BF16
-    t.tune = (p->flags & BRL_CV_WIDE_FORWARD ? 4 : 0) | (p->flags & BRL_CV_NARROW_BACKWARD ? 16 : 0);  // BrlPpoParams.reserved's bits
-    t.batch = p->batch;
-    t.blob = static_cast<const unsigned char*>(b[1]);
-    t.scratch = static_cast<unsigned char*>(b[2]);
-    t.grads = backward ? static_cast<float*>(b[4]) : nullptr;
-    t.grad_sumsq = backward ? head.acc + kCvAccSumsq : nullptr;
-    t.zero = head.acc;
-    t.zero_bytes = 16 * sizeof(double);
-    t.what = what;
-    t.loss_head = cv_loss_head;
-    t.ctx = &head;
-    return launch_train_minibatch(s, t);
-}
+static const char* const kCvInputs[] = {"gain"};
+static const SlParamsHead kCvHead{1, kCvInputs, 1u << 0, BRL_CV_WIDE_FORWARD | BRL_CV_NARROW_BACKWARD, cv_loss_head};
 
 }  // namespace brl
 
@@ -259,11 +168,11 @@ using namespace brl;
 extern "C" {
 
 int32_t brl_cv_grad(brl_stream_t stream, void** b, const void* opaque, size_t len) {
-    return cv_minibatch("brl_cv_grad", (cudaStream_t)stream, b, opaque, len, true);
+    return sl_params_minibatch("brl_cv_grad", true, (cudaStream_t)stream, b, opaque, len, kCvHead);
 }
 
 int32_t brl_cv_eval(brl_stream_t stream, void** b, const void* opaque, size_t len) {
-    return cv_minibatch("brl_cv_eval", (cudaStream_t)stream, b, opaque, len, false);
+    return sl_params_minibatch("brl_cv_eval", false, (cudaStream_t)stream, b, opaque, len, kCvHead);
 }
 
 }  // extern "C"

@@ -1357,3 +1357,40 @@ int32_t brl::launch_train_minibatch(cudaStream_t s, const TrainMinibatch& t) {
     }
     return check_launch(t.what);
 }
+
+int32_t brl::sl_params_minibatch(const char* what, bool backward, cudaStream_t s, void** b, const void* opaque, size_t len,
+                                 const SlParamsHead& head) {
+    if (opaque == nullptr || len != sizeof(BrlSlParams))
+        return fail(BRL_E_OPAQUE, "%s: opaque must be one BrlSlParams (%zu bytes), got %zu", what, sizeof(BrlSlParams), len);
+    const BrlSlParams* p = static_cast<const BrlSlParams*>(opaque);
+    if (p->batch < 0 || p->batch > (1 << 24)) return fail(BRL_E_OPAQUE, "%s: batch must be in [0, 2^24]", what);
+    if (p->batch == 0) return BRL_OK;  // an empty batch is a no-op; its buffers may be NULL
+    const int grads = 3 + head.n_in, stats = grads + (backward ? 1 : 0), acc = stats + 1;  // buffer indices
+    const char* names[16] = {"obs", "blob", "scratch"};
+    for (int k = 0; k < head.n_in; ++k) names[3 + k] = head.in_names[k];
+    if (backward) names[grads] = "grads";
+    names[stats] = "stats";
+    names[acc] = "acc";
+    const int32_t rc = check_buffers(what, b, names, acc + 1, 0, 1u << 0 | 1u << 1 | 1u << 2 | (backward ? 1u << grads : 0u) | 1u << acc);
+    if (rc != BRL_OK) return rc;
+    for (int k = 0; k < head.n_in; ++k)
+        if (((head.in_aligned4 >> k) & 1u) && (reinterpret_cast<uintptr_t>(b[3 + k]) & 3u) != 0)
+            return fail(BRL_E_BUFFER, "%s: %s is not 4-byte aligned", what, head.in_names[k]);
+    const SlHeadCtx ctx{b + 3, static_cast<float*>(b[stats]), static_cast<double*>(b[acc]), p->batch, p->ent_coef, backward};
+    const int32_t tiles = p->flags & head.tile_flags;
+    TrainMinibatch t{};
+    t.obs = b[0];
+    t.obs_flags = p->flags & (BRL_F_OBS_U8 | BRL_F_OBS_BF16);  // same bits as BRL_PPO_OBS_U8 / BRL_PPO_OBS_BF16
+    t.tune = (tiles & BRL_CV_WIDE_FORWARD ? 4 : 0) | (tiles & BRL_CV_NARROW_BACKWARD ? 16 : 0);  // BrlPpoParams.reserved's bits
+    t.batch = p->batch;
+    t.blob = static_cast<const unsigned char*>(b[1]);
+    t.scratch = static_cast<unsigned char*>(b[2]);
+    t.grads = backward ? static_cast<float*>(b[grads]) : nullptr;
+    t.grad_sumsq = backward ? ctx.acc + 14 : nullptr;
+    t.zero = ctx.acc;
+    t.zero_bytes = 16 * sizeof(double);
+    t.what = what;
+    t.loss_head = head.launch;
+    t.ctx = &ctx;
+    return launch_train_minibatch(s, t);
+}

@@ -3,10 +3,8 @@
 // own backward (d loss / d logits, d loss / d value in one pass over the minibatch), and the
 // optimizer step (optax.clip_by_global_norm + optax.adam) over a flat parameter buffer.
 // The MLP forward/backward GEMMs between them are plain library GEMMs (cuBLAS via torch).
-#include <cuda_bf16.h>
-#include <math.h>
-
 #include "common.h"
+#include "loss_head.cuh"
 #include "ppo_gram.cuh"
 
 namespace brl {
@@ -45,17 +43,6 @@ enum { kAccAdv = 0, kAccAdv2, kAccIll, kAccActor, kAccValue, kAccEnt, kAccKl, kA
 static_assert(128 + 40 * 8 <= 512 && 512 + kGramBlocks * kGramN * 4 <= BRL_PPO_SCRATCH_BYTES, "scratch layout");
 static_assert(kAccGramTicket == 13, "gram_args_at (ppo_gram.cuh) places the Gram ticket in f64 13");
 
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-
 // one warp per sample; lane owns actions lane and lane + 32
 struct Row {
     float l[2];
@@ -69,17 +56,7 @@ struct Row {
             legal[k] = in[k] && a.mask[src * kA + j] != 0;
         }
     }
-    // softmax over `sel` entries: returns log-partition; p[k] = probabilities (0 outside sel)
-    __device__ __forceinline__ float softmax(const bool sel[2], float p[2], float logp[2]) const {
-        float mx = warp_max(fmaxf(sel[0] ? l[0] : -INFINITY, sel[1] ? l[1] : -INFINITY));
-        float e0 = sel[0] ? expf(l[0] - mx) : 0.0f, e1 = sel[1] ? expf(l[1] - mx) : 0.0f;
-        float lse = mx + logf(warp_sum(e0 + e1));
-        logp[0] = sel[0] ? l[0] - lse : -INFINITY;
-        logp[1] = sel[1] ? l[1] - lse : -INFINITY;
-        p[0] = sel[0] ? expf(logp[0]) : 0.0f;
-        p[1] = sel[1] ? expf(logp[1]) : 0.0f;
-        return lse;
-    }
+    __device__ __forceinline__ float softmax(const bool sel[2], float p[2], float logp[2]) const { return softmax_sel(l, sel, p, logp); }
 };
 
 // ---- the loss head of K learners at once (brl_ppo_grad_grouped): blockIdx.y = learner --------------------------------
@@ -163,12 +140,6 @@ __global__ void __launch_bounds__(1024) k_ppo_gram_partial(const GramArgs g) {
     pdl_trigger();
     pdl_wait();
     gram_partial<1024>(g, (int)blockIdx.x, (int)gridDim.x, X);
-}
-
-__device__ __forceinline__ void split_store(const PpoArgs& a, int64_t idx, float v) {
-    const __nv_bfloat16 h = __float2bfloat16_rn(v), l = __float2bfloat16_rn(v - __bfloat162float(h));
-    a.dz_hi[idx] = *reinterpret_cast<const unsigned short*>(&h);
-    a.dz_lo[idx] = *reinterpret_cast<const unsigned short*>(&l);
 }
 
 // stats = {total_loss, value_loss, loss_actor, entropy, approx_kl, clipfracs, illegal_action_loss, 0}
@@ -296,9 +267,9 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
             if (ill_grad) d += a.ill_coef * 0.5f * (t_i / sigma) * (qi[k] * v1[k] - q[k] * t_i);
             if constexpr (kAnchored<Anchor...>) d += dkl[k];
             a.dlogits[b * kA + j] = d;
-            if (a.dz_hi) split_store(a, b * 64 + j, d);
+            if (a.dz_hi) store_dz(a.dz_hi, a.dz_lo, b * 64 + j, d);
         }
-        if (a.dz_hi && lane >= 7) split_store(a, b * 64 + 32 + lane, 0.0f);  // columns 39..63 (38 is the value, below)
+        if (a.dz_hi && lane >= 7) store_dz(a.dz_hi, a.dz_lo, b * 64 + 32 + lane, 0.0f);  // columns 39..63 (38 is the value, below)
         if (lane == 0) {
             // value loss (src/update.py:47-72)
             const float v = a.value[b], t = a.targets[src];
@@ -316,7 +287,7 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
                 dv = v - t;
             }
             a.dvalue[b] = a.vf_coef * dv * invB;
-            if (a.dz_hi) split_store(a, b * 64 + 38, a.vf_coef * dv * invB);
+            if (a.dz_hi) store_dz(a.dz_hi, a.dz_lo, b * 64 + 38, a.vf_coef * dv * invB);
             s_actor += (double)loss_actor;
             s_value += (double)vl;
             s_ent += (double)ent;
@@ -326,7 +297,8 @@ __global__ void __launch_bounds__(128) k_ppo_loss(const Args g, int have_prepass
         }
     }
     // block-level sums first (one set of same-address f64 atomics per block, not per warp), then the last block to
-    // arrive (ticket in acc[kAccTicket]) forms the statistics: no separate finalize launch
+    // arrive (ticket in acc[kAccTicket]) forms the statistics: no separate finalize launch.  head_block_sums (loss_head.cuh)
+    // does the same for sums in acc[0..N); these go to scattered slots, and its code with a slot table would differ.
     constexpr int kSums = kAnchored<Anchor...> ? 6 : 5;  // the f64 sums: actor, value, entropy, approx KL, clip fraction (, anchor KL)
     __shared__ double part[4][kSums];
     __shared__ bool last_block;
@@ -489,8 +461,7 @@ static int32_t launch_ppo_chain(cudaStream_t s, const Args& g, PpoArgs& a, int32
     a.value_clipping = (flags & BRL_PPO_VALUE_CLIPPING) != 0;
     a.reward_scaling = (flags & BRL_PPO_REWARD_SCALING) != 0;
     a.masked_policy = (flags & BRL_PPO_UNMASKED_POLICY) == 0;
-    unsigned grid = (unsigned)((a.B + 3) / 4);
-    if (grid > 148u * 8u) grid = 148u * 8u;
+    const unsigned grid = head_grid(a.B);
     const int prepass = a.reward_scaling;
     if (prepass) k_ppo_prepass<Args><<<dim3(grid > 32u ? 32u : grid, K), 128, 0, s>>>(g);
     if (gram) {

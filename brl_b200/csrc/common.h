@@ -89,8 +89,8 @@ struct GramArgs;
 GramArgs gram_args(void** loss_buffers, const BrlPpoParams* p, float* stat);
 int gram_blocks(int64_t batch, int threads);
 
-// One minibatch through the DeepMind MLP on tcgen05 (brl_mlp_train.cu), shared by brl_ppo_grad and brl_sl_grad /
-// brl_sl_eval: gather of the observation, fused forward with the activations kept, the caller's loss head, then (when
+// One minibatch through the DeepMind MLP on tcgen05 (brl_mlp_train.cu), shared by brl_ppo_grad, brl_sl_grad /
+// brl_sl_eval and brl_cv_grad / brl_cv_eval: gather of the observation, fused forward with the activations kept, the caller's loss head, then (when
 // `grads` is set) the fused backward and the bias sums.  The ops differ only in the loss head.
 struct TrainHeadIO {  // what the forward leaves for the loss head, and where the backward reads d loss / d (logits, value)
     const float* logits;  // f32 [B, 38]
@@ -131,6 +131,33 @@ struct TrainMinibatch {
     const TrainGroup* group;     // NULL = one learner
 };
 int32_t launch_train_minibatch(cudaStream_t stream, const TrainMinibatch& t);
+
+// Grid of a warp-per-sample loss head (128 threads, 4 samples a block): one sample per warp, at most 8 blocks per SM of a B200
+inline unsigned head_grid(int64_t batch) {
+    const unsigned grid = (unsigned)((batch + 3) / 4);
+    return grid > 148u * 8u ? 148u * 8u : grid;
+}
+
+// The ops whose opaque is a BrlSlParams (brl_sl_grad / brl_sl_eval, brl_cv_grad / brl_cv_eval): one minibatch through
+// launch_train_minibatch with the head's kernel.  Buffers: [0] obs [1] blob [2] scratch, the head's n_in inputs, then
+// grads (backward only), stats, acc.  obs, blob, scratch, grads and acc are 16-byte aligned.
+struct SlParamsHead {
+    int n_in;              // at most 10
+    const char* const* in_names;
+    unsigned in_aligned4;  // bit k: input k must be 4-byte aligned
+    int32_t tile_flags;    // BrlSlParams.flags bits the op honours: BRL_CV_WIDE_FORWARD / BRL_CV_NARROW_BACKWARD
+    int32_t (*launch)(cudaStream_t, const TrainHeadIO&, const void* ctx);  // ctx: the SlHeadCtx below
+};
+struct SlHeadCtx {
+    void* const* in;  // the head's input buffers
+    float* stats;     // [8]
+    double* acc;      // f64[16], cleared before the forward: the head's sums from 0, |grads|^2 at 14, its ticket at 15
+    int64_t B;
+    float ent_coef;
+    bool backward;    // d loss / d (logits, value) wanted (brl_*_grad)
+};
+int32_t sl_params_minibatch(const char* what, bool backward, cudaStream_t stream, void** buffers, const void* opaque, size_t len,
+                            const SlParamsHead& head);
 
 // brl_ppo_grad_grouped's loss head (brl_ppo.cu): launch_ppo_loss for K learners, one grid row per learner.  Learner k's
 // trajectory buffers are row k of the device table `traj`, its coefficients row k of `coefs`; its forward outputs and

@@ -449,8 +449,7 @@ def ppo_grad(obs, blob, scratch, index, mask, action, old_log_prob, old_value, a
                        illegal_stat=illegal_stat, obs_dtype=obs.dtype)
     if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
         raise _lib.BrlError("ppo_grad: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
-    if grads.dtype != torch.float32 or grads.numel() != L.brl_mlp_num_params():
-        raise _lib.BrlError("ppo_grad: grads must be the flat fp32 gradient buffer")
+    _check_flat_grads("ppo_grad", grads)
     _anchor_args("ppo_grad", anchor_logits, kl_coef)
     p = _lib.BrlPpoParams(B, int(action.numel()), float(clip_eps), float(ent_coef), float(vf_coef), float(illegal_l2_coef),
                           flags, int(tune))
@@ -575,45 +574,11 @@ def sl_acc(device) -> torch.Tensor:
     return torch.zeros(_lib.SL_ACC_BYTES // 8, dtype=torch.float64, device=device)
 
 
-def _sl_params(name, obs, mask, label, scratch, blob, ent_coef):
+def _head_params(name, B, obs, scratch, blob, ent_coef, tiles=0):
+    """obs as the loss-head ops on BrlSlParams read it (bool as uint8), and their params; after the op's own input checks"""
     L = _lib.load()
-    B = int(label.shape[0])
     if obs.dtype == torch.bool:
         obs = obs.view(torch.uint8)
-    if label.dtype != torch.int32 or mask.dtype != torch.uint8:
-        raise _lib.BrlError(f"{name}: label must be int32 and mask uint8")
-    if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
-        raise _lib.BrlError(f"{name}: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
-    return obs, _lib.BrlSlParams(B, float(ent_coef), obs_flag(obs.dtype))
-
-
-def sl_grad(obs, blob, scratch, mask, label, grads, stats, acc, *, ent_coef=0.0) -> None:
-    """One minibatch of value_and_grad(loss) of sl.py:169-184 through the MLP on tcgen05 -> flat fp32 gradients and
-    stats[:5] = {total_loss, target_loss, entropy, accuracy, illegal_actions_prob} of the parameters before the step."""
-    obs, p = _sl_params("sl_grad", obs, mask, label, scratch, blob, ent_coef)
-    if grads.dtype != torch.float32 or grads.numel() != _lib.load().brl_mlp_num_params():
-        raise _lib.BrlError("sl_grad: grads must be the flat fp32 gradient buffer")
-    _call("brl_sl_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(grads), _ptr(stats), _ptr(acc)], p)
-
-
-def sl_eval(obs, blob, scratch, mask, label, stats, acc, *, ent_coef=0.0) -> None:
-    """sl_grad's statistics without the backward (accuracy, sl.py:186-194; test metrics, sl.py:288-301)."""
-    obs, p = _sl_params("sl_eval", obs, mask, label, scratch, blob, ent_coef)
-    _call("brl_sl_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(stats), _ptr(acc)], p)
-
-
-CV_WIDE_FORWARD, CV_NARROW_BACKWARD = 1 << 16, 1 << 17  # brl_cv_grad's tile-width experiment bits (BRL_CV_*)
-
-
-def _cv_params(name, obs, gain, scratch, blob, ent_coef, tiles=0):
-    L = _lib.load()
-    B = int(gain.shape[0])
-    if obs.dtype == torch.bool:
-        obs = obs.view(torch.uint8)
-    if gain.dtype != torch.float32 or tuple(gain.shape) != (B, NUM_ACTIONS):
-        raise _lib.BrlError(f"{name}: gain must be float32 [B, 38] (NaN for an illegal call)")
-    if tuple(obs.shape) != (B, OBS_DIM):
-        raise _lib.BrlError(f"{name}: obs must be [B, 480] with B = gain.shape[0]")
     if scratch.numel() < L.brl_mlp_train_scratch_bytes(B) or blob.numel() < L.brl_mlp_train_blob_bytes():
         raise _lib.BrlError(f"{name}: scratch / blob too small (ops.mlp_train_scratch, ops.mlp_pack_train)")
     if tiles & ~(CV_WIDE_FORWARD | CV_NARROW_BACKWARD):
@@ -621,20 +586,58 @@ def _cv_params(name, obs, gain, scratch, blob, ent_coef, tiles=0):
     return obs, _lib.BrlSlParams(B, float(ent_coef), obs_flag(obs.dtype) | tiles)
 
 
+def _check_flat_grads(name, grads):
+    if grads.dtype != torch.float32 or grads.numel() != _lib.load().brl_mlp_num_params():
+        raise _lib.BrlError(f"{name}: grads must be the flat fp32 gradient buffer")
+
+
+def _check_sl_inputs(name, mask, label):
+    if label.dtype != torch.int32 or mask.dtype != torch.uint8:
+        raise _lib.BrlError(f"{name}: label must be int32 and mask uint8")
+
+
+def sl_grad(obs, blob, scratch, mask, label, grads, stats, acc, *, ent_coef=0.0) -> None:
+    """One minibatch of value_and_grad(loss) of sl.py:169-184 through the MLP on tcgen05 -> flat fp32 gradients and
+    stats[:5] = {total_loss, target_loss, entropy, accuracy, illegal_actions_prob} of the parameters before the step."""
+    _check_sl_inputs("sl_grad", mask, label)
+    obs, p = _head_params("sl_grad", int(label.shape[0]), obs, scratch, blob, ent_coef)
+    _check_flat_grads("sl_grad", grads)
+    _call("brl_sl_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(grads), _ptr(stats), _ptr(acc)], p)
+
+
+def sl_eval(obs, blob, scratch, mask, label, stats, acc, *, ent_coef=0.0) -> None:
+    """sl_grad's statistics without the backward (accuracy, sl.py:186-194; test metrics, sl.py:288-301)."""
+    _check_sl_inputs("sl_eval", mask, label)
+    obs, p = _head_params("sl_eval", int(label.shape[0]), obs, scratch, blob, ent_coef)
+    _call("brl_sl_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(mask), _ptr(label), _ptr(stats), _ptr(acc)], p)
+
+
+CV_WIDE_FORWARD, CV_NARROW_BACKWARD = 1 << 16, 1 << 17  # brl_cv_grad's tile-width experiment bits (BRL_CV_*)
+
+
+def _check_cv_inputs(name, obs, gain):
+    B = int(gain.shape[0])
+    if gain.dtype != torch.float32 or tuple(gain.shape) != (B, NUM_ACTIONS):
+        raise _lib.BrlError(f"{name}: gain must be float32 [B, 38] (NaN for an illegal call)")
+    if tuple(obs.shape) != (B, OBS_DIM):
+        raise _lib.BrlError(f"{name}: obs must be [B, 480] with B = gain.shape[0]")
+
+
 def cv_grad(obs, blob, scratch, gain, grads, stats, acc, *, ent_coef=0.0, tiles=0) -> None:
     """One minibatch of the call-value policy-improvement loss (DESIGN.md f17) through the MLP on tcgen05: gain f32[B, 38]
     (IMPs, NaN = illegal), loss = -mean(sum_a pi_a g_a) / 24 - ent_coef * mean entropy -> flat fp32 gradients, stats[8]
     (include/brl_b200.h brl_cv_grad) and acc[14] = sum of squares of the gradient (sl_acc's buffer).  `tiles`: the
     CV_WIDE_FORWARD / CV_NARROW_BACKWARD experiment bits (0: the measured tile widths)."""
-    obs, p = _cv_params("cv_grad", obs, gain, scratch, blob, ent_coef, tiles)
-    if grads.dtype != torch.float32 or grads.numel() != _lib.load().brl_mlp_num_params():
-        raise _lib.BrlError("cv_grad: grads must be the flat fp32 gradient buffer")
+    _check_cv_inputs("cv_grad", obs, gain)
+    obs, p = _head_params("cv_grad", int(gain.shape[0]), obs, scratch, blob, ent_coef, tiles)
+    _check_flat_grads("cv_grad", grads)
     _call("brl_cv_grad", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(gain), _ptr(grads), _ptr(stats), _ptr(acc)], p)
 
 
 def cv_eval(obs, blob, scratch, gain, stats, acc, *, ent_coef=0.0, tiles=0) -> None:
     """cv_grad's statistics without the backward (bit-equal to cv_grad's on the same inputs)."""
-    obs, p = _cv_params("cv_eval", obs, gain, scratch, blob, ent_coef, tiles)
+    _check_cv_inputs("cv_eval", obs, gain)
+    obs, p = _head_params("cv_eval", int(gain.shape[0]), obs, scratch, blob, ent_coef, tiles)
     _call("brl_cv_eval", [_ptr(obs), _ptr(blob), _ptr(scratch), _ptr(gain), _ptr(stats), _ptr(acc)], p)
 
 
