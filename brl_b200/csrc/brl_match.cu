@@ -8,21 +8,24 @@
 //                         the branches played out by a nested WHILE node (DESIGN.md f16); optionally each decision's
 //                         observation and gains as training examples (DESIGN.md f17)
 //
-//   init (brl_init) -> Table_info A / B (brl_state_fields) -> grouping (brl_model_rows) -> control
+//   match start: init (brl_init) -> Table_info A / B (brl_state_fields)
+//   grouping (brl_model_rows) -> control
 //   WHILE (control said so) {
 //       [path kernel -> IF fused forward / IF per-layer forward]    the grouped forward, sized from the device count
 //       [brl_system_stats] -> brl_duplicate_step -> cum_return += rewards[:, 0] -> grouping -> control
 //   }
 //   match sums (brl_match_stats_ranges, or brl_match_stats for one range)
 //
-// brl_evaluate_match runs the same skeleton: its body adds brl_eval_act_log after the forward (full statistics), steps with
-// brl_step instead of brl_duplicate_step where there is one table, and ends with brl_eval_summary (or nothing: simple).
+// All three ops share the match start and the loop (emit_while: grouping, control and a WHILE node whose body ends in
+// grouping and control).  brl_evaluate_match's body adds brl_eval_act_log after the forward (full statistics), steps with
+// brl_step instead of brl_duplicate_step where there is one table, and the op ends with brl_eval_summary (or nothing:
+// simple).  brl_call_values' body runs a second such loop, over the branch batch, between the forward and the step.
 //
 // The control kernel reads the padded row count brl_model_rows left in offsets[M] and sets the loop's condition: the loop
-// ends when no env is live, when a live env's net id is outside [0, M), or at BRL_MATCH_MAX_STEPS forwards; the last two
-// write a status.  Nothing is read back to the host.  The forward path follows the host's rule (fused from kPairMinM rows
-// on, per-layer below, unless BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED pin it), applied to the device count by a
-// path kernel and two IF nodes.
+// ends when no env is live, when a live env's net id is outside [0, M), at the loop's bound (BRL_MATCH_MAX_STEPS forwards
+// for a match), or once a loop of the graph has failed; the first two failures write a status.  Nothing is read back to the
+// host.  The forward path follows the host's rule (fused from kPairMinM rows on, per-layer below, unless
+// BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED pin it), applied to the device count by a path kernel and two IF nodes.
 //
 // On a plain stream the graph is captured on a private stream, instantiated once per set of buffers and parameters
 // (cached), and launched.  On a stream that is being captured (torch.cuda.graph, an XLA command buffer) the same nodes
@@ -101,15 +104,16 @@ __global__ void __launch_bounds__(256) k_sum_rewards(float* __restrict__ cum_ret
     cum_return[i] += r.x;
 }
 
-// after each grouping: continue while rows are live; stop with a status on a bad net id or at the step bound.  `iter` counts
-// the forwards the loop has been allowed to run.
+// after each grouping: continue while rows are live; stop with a status on a bad net id or at the step bound, and stop once a
+// loop of the graph has failed (brl_call_values' two loops share the status; a BRL_MATCH_RECORD_CAPACITY status does not stop
+// them: the sums stay complete).  `iter` counts the forwards the loop has been allowed to run.
 __global__ void k_match_control(const int32_t* __restrict__ n_rows, int32_t* __restrict__ iter, int32_t* __restrict__ status,
-                                cudaGraphConditionalHandle loop) {
-    const int rows = *n_rows, it = *iter;
-    bool go = rows > 0;
+                                cudaGraphConditionalHandle loop, int bound) {
+    const int rows = *n_rows, it = *iter, st = *status;
+    bool go = rows > 0 && st != BRL_MATCH_BAD_MODEL && st != BRL_MATCH_STEP_BOUND;
     if (rows < 0) {
         *status = BRL_MATCH_BAD_MODEL;
-    } else if (go && it >= BRL_MATCH_MAX_STEPS) {
+    } else if (go && it >= bound) {
         *status = BRL_MATCH_STEP_BOUND;
         go = false;
     }
@@ -125,22 +129,6 @@ __global__ void k_match_path(const int32_t* __restrict__ n_rows, cudaGraphCondit
 }
 
 // ---- brl_call_values (env_device.cuh, DESIGN.md f16) ----------------------------------------------------------------------
-// the loop condition of brl_call_values' two loops: like k_match_control with the bound a parameter, and a stop once a loop
-// has failed (a BRL_MATCH_RECORD_CAPACITY status does not stop the loops: the sums stay complete)
-__global__ void k_cv_control(const int32_t* __restrict__ n_rows, int32_t* __restrict__ iter, int32_t* __restrict__ status,
-                             cudaGraphConditionalHandle loop, int bound) {
-    const int rows = *n_rows, it = *iter, st = *status;
-    bool go = rows > 0 && st != BRL_MATCH_BAD_MODEL && st != BRL_MATCH_STEP_BOUND;
-    if (rows < 0) {
-        *status = BRL_MATCH_BAD_MODEL;
-    } else if (go && it >= bound) {
-        *status = BRL_MATCH_STEP_BOUND;
-        go = false;
-    }
-    if (go) *iter = it + 1;
-    cudaGraphSetConditional(loop, go ? 1u : 0u);
-}
-
 // one thread per branch slot j = 38 i + a of base env i: the slot's state is S_i, to be stepped with call a by brl_step; a
 // slot whose env is finished or whose call is illegal is born finished (a no-op step, never listed by brl_model_rows).  The
 // slot's nets by player id come from the env's (by team: expanded); r[j] = 0; the slot loop's iteration counter restarts.
@@ -367,8 +355,8 @@ static int32_t model_rows(const MatchPlan& q, cudaStream_t s) {
     return brl_model_rows(s, b, &p, sizeof(p));
 }
 
-static int32_t control(const MatchPlan& q, cudaStream_t s, cudaGraphConditionalHandle loop) {
-    k_match_control<<<1, 1, 0, s>>>(q.offsets() + q.M, q.at<int32_t>(q.L.ctl), q.status, loop);
+static int32_t control(const MatchPlan& q, cudaStream_t s, cudaGraphConditionalHandle loop, int bound) {
+    k_match_control<<<1, 1, 0, s>>>(q.offsets() + q.M, q.at<int32_t>(q.L.ctl), q.status, loop, bound);
     return launched(q.who, "control");
 }
 
@@ -417,6 +405,23 @@ static int32_t capture_into(const char* who, cudaGraph_t body, cudaStream_t side
     return BRL_OK;
 }
 
+// a loop over q's envs on s: grouping and control, then a WHILE node whose body (captured on s_body) is what `body` enqueues
+// followed by grouping and control.  The loop runs at most `bound` times.
+template <class F>
+static int32_t emit_while(const MatchPlan& q, cudaStream_t s, cudaStream_t s_body, int bound, F&& body) {
+    int32_t rc;
+    cudaGraphConditionalHandle loop;
+    cudaGraph_t g;
+    if ((rc = new_handle(q.who, s, &loop)) || (rc = model_rows(q, s)) || (rc = control(q, s, loop, bound)) ||
+        (rc = add_conditional(q.who, s, loop, cudaGraphCondTypeWhile, &g)))
+        return rc;
+    return capture_into(q.who, g, s_body, [&](cudaStream_t sb) {
+        int32_t r;
+        if ((r = body(sb)) || (r = model_rows(q, sb))) return r;
+        return control(q, sb, loop, bound);
+    });
+}
+
 static int32_t forward(const MatchPlan& q, cudaStream_t s, int32_t path_flag) {
     const int32_t flags = (q.flags & BRL_F_MLP_BF16) | path_flag;
     return launch_policy_grouped(s, flags, q.cap, q.M, q.obs, q.pool, q.at<unsigned char>(q.L.forward), static_cast<uint8_t*>(q.mask),
@@ -424,17 +429,19 @@ static int32_t forward(const MatchPlan& q, cudaStream_t s, int32_t path_flag) {
                                  q.offsets() + q.M, q.logits);
 }
 
-// the env step of one iteration: brl_duplicate_step on both tables (:164, :772-774), or brl_step without auto-reset (:406;
-// make_simple_evaluate: src/utils.py:133-202 one sub-step at a time)
-static int32_t env_step(const MatchPlan& q, cudaStream_t s) {
+// brl_step without auto-reset on one table (:406; make_simple_evaluate: src/utils.py:133-202 one sub-step at a time)
+static int32_t table_step(const MatchPlan& q, cudaStream_t s) {
     const BrlParams p = env_params(q, q.n);
-    void* const action = q.at(q.L.action);
-    if (q.mode == BRL_EVAL_MATCH_SINGLE || q.mode == BRL_EVAL_MATCH_SIMPLE) {
-        void* b[10] = {q.state, action, const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated, q.player,
-                       nullptr};
-        return brl_step(s, b, &p, sizeof(p));
-    }
-    void* b[21] = {q.state, action, const_cast<void*>(q.table)};
+    void* b[10] = {q.state, q.at(q.L.action), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
+                   q.player, nullptr};
+    return brl_step(s, b, &p, sizeof(p));
+}
+
+// the env step of one iteration: brl_duplicate_step on both tables (:164, :772-774), or one table's step
+static int32_t env_step(const MatchPlan& q, cudaStream_t s) {
+    if (q.mode == BRL_EVAL_MATCH_SINGLE || q.mode == BRL_EVAL_MATCH_SIMPLE) return table_step(q, s);
+    const BrlParams p = env_params(q, q.n);
+    void* b[21] = {q.state, q.at(q.L.action), const_cast<void*>(q.table)};
     for (int t = 0; t < 2; ++t)
         for (int k = 0; k < 6; ++k) b[3 + 6 * t + k] = q.info[t][k];
     b[15] = q.state;
@@ -466,7 +473,7 @@ static int32_t emit_forward(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2
     return BRL_OK;
 }
 
-static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, cudaGraphConditionalHandle loop) {
+static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2) {
     int32_t rc = emit_forward(q, s1, s2);
     if (rc != BRL_OK) return rc;
     if (q.acc) {  // the acting team's masked argmax and update_log_info; free-run: team 2 passes, its forwarded rows unread
@@ -490,9 +497,7 @@ static int32_t emit_body(const MatchPlan& q, cudaStream_t s1, cudaStream_t s2, c
         k_sum_rewards<<<blocks(q.n), 256, 0, s1>>>(q.cum_return, reinterpret_cast<float4*>(q.rewards_sum), q.at<float4>(q.L.rewards), q.n);
     else
         k_add_reward<<<blocks(q.n), 256, 0, s1>>>(q.cum_return, q.at<float4>(q.L.rewards), q.n);
-    if ((rc = launched(q.who, "cum_return"))) return rc;
-    if ((rc = model_rows(q, s1))) return rc;
-    return control(q, s1, loop);
+    return launched(q.who, "cum_return");
 }
 
 // brl_evaluate_match's end: the final state's fields and every log_info sum (src/evaluation.py:448-596, :839-1027)
@@ -527,11 +532,30 @@ static int32_t emit_summary(const MatchPlan& q, cudaStream_t s) {
     return brl_eval_summary(s, bs, &ps, sizeof(ps));
 }
 
+// the envs from the keys (src/evaluation.py:93-95, observation in bf16: what the forward reads) and, where the plan has
+// Table_infos, Table_info A = B = the init state's terminated, rewards, last_bid, last_bidder, call_x, call_xx (:97-112)
+static int32_t match_start(const MatchPlan& q, cudaStream_t s) {
+    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
+                   q.player};
+    const BrlParams p = env_params(q, q.n);
+    int32_t rc;
+    if ((rc = brl_init(s, bi, &p, sizeof(p)))) return rc;
+    if (q.mode != 0 && q.mode != BRL_EVAL_MATCH_DUPLICATE) return BRL_OK;
+    void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
+    if ((rc = brl_state_fields(s, bf, &p, sizeof(p)))) return rc;
+    const size_t un = (size_t)q.n, bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
+    if (cudaMemcpyAsync(q.info[0][0], q.terminated, bytes[0], cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+        cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+        return launched(q.who, "Table_info");
+    for (int k = 0; k < 6; ++k)
+        if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+            return launched(q.who, "Table_info");
+    return BRL_OK;
+}
+
 // the whole match on the capturing stream s0 (its own capture, or the caller's)
 static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, cudaStream_t s2) {
     int32_t rc;
-    cudaGraphConditionalHandle loop;
-    if ((rc = new_handle(q.who, s0, &loop))) return rc;
     const size_t un = (size_t)q.n;
     if (cudaMemsetAsync(q.status, 0, sizeof(int32_t), s0) != cudaSuccess ||
         cudaMemsetAsync(q.at(q.L.ctl), 0, sizeof(int32_t), s0) != cudaSuccess ||
@@ -546,11 +570,7 @@ static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, 
         k_player_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.free_run ? make_int4(0, 2, 0, 0) : make_int4(0, 2, 1, 1), q.n);
     else if (q.default_models)
         k_pair_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.n);
-    // src/evaluation.py:93-95: the envs from the given keys, observation in bf16 (what the forward reads)
-    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
-                   q.player};
-    BrlParams p = env_params(q, q.n);
-    if ((rc = brl_init(s0, bi, &p, sizeof(p)))) return rc;
+    if ((rc = match_start(q, s0))) return rc;
     if (q.mode == BRL_EVAL_MATCH_SIMPLE) {
         if (q.partner)
             k_actor_partner_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player),
@@ -559,23 +579,7 @@ static int32_t emit_match(const MatchPlan& q, cudaStream_t s0, cudaStream_t s1, 
             k_actor_models<<<blocks(q.n), 256, 0, s0>>>(q.env_models, q.at<int8_t>(q.L.actor), static_cast<const int8_t*>(q.player), q.n);
         if ((rc = launched(q.who, "actor"))) return rc;
     }
-    if (q.mode == 0 || q.mode == BRL_EVAL_MATCH_DUPLICATE) {
-        // :97-112 Table_info A = B = the init state's terminated, rewards, last_bid, last_bidder, call_x, call_xx
-        void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
-        if ((rc = brl_state_fields(s0, bf, &p, sizeof(p)))) return rc;
-        const size_t bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
-        if (cudaMemcpyAsync(q.info[0][0], q.terminated, bytes[0], cudaMemcpyDeviceToDevice, s0) != cudaSuccess ||
-            cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-            return launched(q.who, "Table_info");
-        for (int k = 0; k < 6; ++k)
-            if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-                return launched(q.who, "Table_info");
-    }
-    if ((rc = model_rows(q, s0)) || (rc = control(q, s0, loop))) return rc;
-    cudaGraph_t body;
-    if ((rc = add_conditional(q.who, s0, loop, cudaGraphCondTypeWhile, &body)) ||
-        (rc = capture_into(q.who, body, s1, [&](cudaStream_t s) { return emit_body(q, s, s2, loop); })))
-        return rc;
+    if ((rc = emit_while(q, s0, s1, BRL_MATCH_MAX_STEPS, [&](cudaStream_t s) { return emit_body(q, s, s2); }))) return rc;
     if (q.mode == BRL_EVAL_MATCH_SIMPLE) return BRL_OK;  // the output is R itself
     if (q.mode != 0) return emit_summary(q, s0);
     // :199-201 the match sums, per range
@@ -694,7 +698,17 @@ static MatchPlan base_plan(const char* who, int mode, const BrlParams* p, int64_
     return q;
 }
 
-static bool misaligned(const void* ptr, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(ptr) & (bytes - 1)) != 0; }
+// how many of b[from, to) are given: an all-or-none group has none or to - from
+static int given(void* const* b, int from, int to) {
+    int k = 0;
+    for (int i = from; i < to; ++i) k += b[i] != nullptr;
+    return k;
+}
+
+// the names of a Table_info A / B pair of buffers, in buffer order
+#define BRL_TABLE_INFO_NAMES                                                                                                  \
+    "table_a.terminated", "table_a.rewards", "table_a.last_bid", "table_a.last_bidder", "table_a.call_x", "table_a.call_xx",  \
+        "table_b.terminated", "table_b.rewards", "table_b.last_bid", "table_b.last_bidder", "table_b.call_x", "table_b.call_xx"
 
 // ---- brl_call_values ----------------------------------------------------------------------------------------------------
 constexpr int kAuctionMaxCalls = BRL_MATCH_MAX_STEPS / 2;  // the bound of one branch's auction
@@ -715,26 +729,18 @@ struct CvPlan {
     unsigned long long* saved;  // the record count before the iteration's gains: a spare word of the base loop's ctl
 };
 
-// brl_step without auto-reset on the branch batch, then r += rewards[:, 0] (non-zero on a slot's last step only)
+// one step of the branch batch, then r += rewards[:, 0] (non-zero on a slot's last step only)
 static int32_t branch_step(const CvPlan& c, cudaStream_t s) {
     const MatchPlan& br = c.br;
-    const BrlParams p = env_params(br, br.n);
-    void* b[10] = {br.state, br.at(br.L.action), const_cast<void*>(br.table), br.state, br.obs, br.mask, br.at(br.L.rewards),
-                   br.terminated, br.player, nullptr};
     int32_t rc;
-    if ((rc = brl_step(s, b, &p, sizeof(p)))) return rc;
+    if ((rc = table_step(br, s))) return rc;
     k_add_reward<<<blocks(br.n), 256, 0, s>>>(c.r, br.at<float4>(br.L.rewards), br.n);
     return launched(br.who, "branch reward");
 }
 
-static int32_t cv_control(const MatchPlan& q, cudaStream_t s, cudaGraphConditionalHandle loop, int bound) {
-    k_cv_control<<<1, 1, 0, s>>>(q.offsets() + q.M, q.at<int32_t>(q.L.ctl), q.status, loop, bound);
-    return launched(q.who, "control");
-}
-
 // one base iteration: forward -> branch every live env on every legal call -> play the branches out (nested WHILE) -> gains
-// -> brl_duplicate_step -> grouping -> control
-static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, cudaStream_t s3, cudaGraphConditionalHandle loop) {
+// -> brl_duplicate_step
+static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, cudaStream_t s3) {
     const MatchPlan &q = c.q, &br = c.br;
     int32_t rc;
     if ((rc = emit_forward(q, s1, s2))) return rc;
@@ -746,17 +752,12 @@ static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, c
     else
         k_branch_calls<2><<<blocks(br.n), 256, 0, s1>>>(state, done, q.env_models, static_cast<uint4*>(br.state), br.at<int32_t>(br.L.action),
                                                        reinterpret_cast<int4*>(br.env_models), c.r, br.at<int32_t>(br.L.ctl), q.n);
-    cudaGraphConditionalHandle inner;
-    if ((rc = launched(q.who, "branch calls")) || (rc = branch_step(c, s1)) || (rc = model_rows(br, s1)) ||
-        (rc = new_handle(q.who, s1, &inner)) || (rc = cv_control(br, s1, inner, kAuctionMaxCalls)))
-        return rc;
     // the branches' auctions to their ends: the forward's IF nodes sit one level deeper here, in the nested WHILE's body
-    cudaGraph_t body;
-    if ((rc = add_conditional(q.who, s1, inner, cudaGraphCondTypeWhile, &body)) ||
-        (rc = capture_into(q.who, body, s2, [&](cudaStream_t s) {
+    if ((rc = launched(q.who, "branch calls")) || (rc = branch_step(c, s1)) ||
+        (rc = emit_while(br, s1, s2, kAuctionMaxCalls, [&](cudaStream_t s) {
              int32_t r2;
-             if ((r2 = emit_forward(br, s, s3)) || (r2 = branch_step(c, s)) || (r2 = model_rows(br, s))) return r2;
-             return cv_control(br, s, inner, kAuctionMaxCalls);
+             if ((r2 = emit_forward(br, s, s3))) return r2;
+             return branch_step(c, s);
          })))
         return rc;
     const int32_t* action = q.at<int32_t>(q.L.action);
@@ -769,17 +770,15 @@ static int32_t emit_cv_body(const CvPlan& c, cudaStream_t s1, cudaStream_t s2, c
     if (c.ex_obs)  // at most one record per base env and iteration: n warps
         k_cv_examples<<<blocks(q.n * 32), 256, 0, s1>>>(static_cast<const uint4*>(q.obs), c.ra, c.rb, c.o, c.saved, c.ex_obs,
                                                          c.ex_gain);
-    if ((rc = launched(q.who, "gains")) || (rc = env_step(q, s1)) || (rc = model_rows(q, s1))) return rc;
-    return cv_control(q, s1, loop, BRL_MATCH_MAX_STEPS);
+    if ((rc = launched(q.who, "gains"))) return rc;
+    return env_step(q, s1);
 }
 
-// the whole op on s0: zeroed outputs, init and Table_info A = B as brl_duplicate_match, then the base loop
+// the whole op on s0: zeroed outputs, the match start of brl_duplicate_match, then the base loop
 static int32_t emit_call_values(const CvPlan& c, cudaStream_t s0, cudaStream_t s1, cudaStream_t s2, cudaStream_t s3) {
     const MatchPlan& q = c.q;
     const size_t un = (size_t)q.n, cells = (size_t)q.M * kSysContexts * kNumActions * kNumActions * kCvStats * 8;
     int32_t rc;
-    cudaGraphConditionalHandle loop;
-    if ((rc = new_handle(q.who, s0, &loop))) return rc;
     if (cudaMemsetAsync(q.status, 0, sizeof(int32_t), s0) != cudaSuccess ||
         cudaMemsetAsync(q.at(q.L.ctl), 0, sizeof(int32_t), s0) != cudaSuccess ||
         cudaMemsetAsync(q.at(q.L.action), 0, un * sizeof(int32_t), s0) != cudaSuccess ||
@@ -788,23 +787,8 @@ static int32_t emit_call_values(const CvPlan& c, cudaStream_t s0, cudaStream_t s
         cudaMemsetAsync(c.o.mismatch, 0, (size_t)q.M * 8, s0) != cudaSuccess ||
         (c.o.count && cudaMemsetAsync(c.o.count, 0, 8, s0) != cudaSuccess))
         return launched(q.who, "memset");
-    void* bi[8] = {const_cast<void*>(q.keys), const_cast<void*>(q.table), q.state, q.obs, q.mask, q.at(q.L.rewards), q.terminated,
-                   q.player};
-    BrlParams p = env_params(q, q.n);
-    if ((rc = brl_init(s0, bi, &p, sizeof(p)))) return rc;
-    void* bf[12] = {q.state, nullptr, nullptr, nullptr, nullptr, q.info[0][2], q.info[0][3], q.info[0][4], q.info[0][5]};
-    if ((rc = brl_state_fields(s0, bf, &p, sizeof(p)))) return rc;
-    const size_t bytes[6] = {un, un * 16, un * 4, un * 4, un, un};
-    if (cudaMemcpyAsync(q.info[0][0], q.terminated, bytes[0], cudaMemcpyDeviceToDevice, s0) != cudaSuccess ||
-        cudaMemcpyAsync(q.info[0][1], q.at(q.L.rewards), bytes[1], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-        return launched(q.who, "Table_info");
-    for (int k = 0; k < 6; ++k)
-        if (cudaMemcpyAsync(q.info[1][k], q.info[0][k], bytes[k], cudaMemcpyDeviceToDevice, s0) != cudaSuccess)
-            return launched(q.who, "Table_info");
-    if ((rc = model_rows(q, s0)) || (rc = cv_control(q, s0, loop, BRL_MATCH_MAX_STEPS))) return rc;
-    cudaGraph_t body;
-    if ((rc = add_conditional(q.who, s0, loop, cudaGraphCondTypeWhile, &body))) return rc;
-    return capture_into(q.who, body, s1, [&](cudaStream_t s) { return emit_cv_body(c, s, s2, s3, loop); });
+    if ((rc = match_start(q, s0))) return rc;
+    return emit_while(q, s0, s1, BRL_MATCH_MAX_STEPS, [&](cudaStream_t s) { return emit_cv_body(c, s, s2, s3); });
 }
 
 }  // namespace brl
@@ -839,21 +823,13 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     if (p->n_envs > INT32_MAX / 2) return fail(BRL_E_OPAQUE, "brl_duplicate_match: n_envs too large");
     if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_duplicate_match: n_deals must be > 0");
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_duplicate_match: sampling is not supported (argmax only)");
-    BRL_REQUIRE(b[0], "keys");
-    BRL_REQUIRE(b[1], "deal_table");
-    BRL_REQUIRE(b[2], "pool");
-    if (b[3] != nullptr && (reinterpret_cast<uintptr_t>(b[3]) & 7u)) return fail(BRL_E_BUFFER, "brl_duplicate_match: env_models is misaligned");
-    if (b[4] != nullptr && (reinterpret_cast<uintptr_t>(b[4]) & 7u)) return fail(BRL_E_BUFFER, "brl_duplicate_match: range offsets are misaligned");
-    BRL_REQUIRE(b[5], "scratch");
-    if (b[6] == nullptr || (reinterpret_cast<uintptr_t>(b[6]) & 3u)) return fail(BRL_E_BUFFER, "brl_duplicate_match: cum_return is NULL or misaligned");
-    if (b[7] == nullptr || (reinterpret_cast<uintptr_t>(b[7]) & 7u)) return fail(BRL_E_BUFFER, "brl_duplicate_match: sums is NULL or misaligned");
-    if (b[8] == nullptr || (reinterpret_cast<uintptr_t>(b[8]) & 3u)) return fail(BRL_E_BUFFER, "brl_duplicate_match: status is NULL or misaligned");
-    int given = 0;
-    for (int k = 9; k < 21; ++k) given += b[k] != nullptr;
-    if (given != 0 && given != 12) return fail(BRL_E_BUFFER, "brl_duplicate_match: give all twelve Table_info buffers [9..20] or none");
-    if (given && ((reinterpret_cast<uintptr_t>(b[10]) | reinterpret_cast<uintptr_t>(b[16])) & 15u))
-        return fail(BRL_E_BUFFER, "brl_duplicate_match: Table_info rewards are not 16-byte aligned");
-    if (misaligned(b[21], 4)) return fail(BRL_E_BUFFER, "brl_duplicate_match: the system histogram [21] is not 4-byte aligned");
+    static const char* names[22] = {"keys", "deal_table", "pool", "env_models", "range offsets", "scratch", "cum_return", "sums",
+                                    "status", BRL_TABLE_INFO_NAMES, "system histogram [21]"};
+    static const uint8_t align[22] = {16, 16, 16, 8, 8, 16, 4, 8, 4, 0, 16, 0, 0, 0, 0, 0, 16, 0, 0, 0, 0, 4};
+    const unsigned nullable = 1u << 3 | 1u << 4 | 0xFFFu << 9 | 1u << 21;
+    if ((rc = check_buffers("brl_duplicate_match", b, names, 22, nullable, 0u, align))) return rc;
+    const int tables = given(b, 9, 21);
+    if (tables != 0 && tables != 12) return fail(BRL_E_BUFFER, "brl_duplicate_match: give all twelve Table_info buffers [9..20] or none");
 
     MatchPlan q = base_plan("brl_duplicate_match", 0, p, M, b[5]);
     q.P = P;
@@ -864,7 +840,7 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
     q.cum_return = static_cast<float*>(b[6]);
     q.sums = static_cast<double*>(b[7]);
     q.status = static_cast<int32_t*>(b[8]);
-    if (given)
+    if (tables)
         for (int t = 0; t < 2; ++t)
             for (int k = 0; k < 6; ++k) q.info[t][k] = b[9 + 6 * t + k];
     q.default_models = b[3] == nullptr;
@@ -900,27 +876,19 @@ int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, si
     if (p->n_envs > INT32_MAX / 2) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_envs too large");
     if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_evaluate_match: n_deals must be > 0");
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_evaluate_match: sampling is not supported (argmax only)");
-    BRL_REQUIRE(b[0], "keys");
-    BRL_REQUIRE(b[1], "deal_table");
-    BRL_REQUIRE(b[2], "pool");
-    BRL_REQUIRE(b[3], "scratch");
-    if (b[4] == nullptr || misaligned(b[4], 4)) return fail(BRL_E_BUFFER, "brl_evaluate_match: cum_return is NULL or misaligned");
-    if (full && (b[5] == nullptr || misaligned(b[5], 4))) return fail(BRL_E_BUFFER, "brl_evaluate_match: acc is NULL or misaligned");
-    if (full && (b[6] == nullptr || misaligned(b[6], 8))) return fail(BRL_E_BUFFER, "brl_evaluate_match: sums is NULL or misaligned");
-    if (b[7] == nullptr || misaligned(b[7], 4)) return fail(BRL_E_BUFFER, "brl_evaluate_match: status is NULL or misaligned");
-    int tables = 0, finals = 0;
-    for (int k = 8; k < 20; ++k) tables += b[k] != nullptr;
-    for (int k = 20; k < 26; ++k) finals += b[k] != nullptr;
-    if (mode == BRL_EVAL_MATCH_DUPLICATE) {
-        if (tables != 0 && tables != 12) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all twelve Table_info buffers [8..19] or none");
-        if (tables && (misaligned(b[9], 16) || misaligned(b[15], 16)))
-            return fail(BRL_E_BUFFER, "brl_evaluate_match: Table_info rewards are not 16-byte aligned");
-    }
-    if (mode == BRL_EVAL_MATCH_SINGLE) {
-        if (finals != 0 && finals != 6) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all six final-state buffers [20..25] or none");
-        if (finals && (misaligned(b[20], 16) || misaligned(b[21], 16) || misaligned(b[22], 2) || misaligned(b[23], 16)))
-            return fail(BRL_E_BUFFER, "brl_evaluate_match: the final state, observation or rewards are not 16-byte aligned (mask: 2)");
-    }
+    // buffers a mode does not read are not checked: acc and sums in simple mode, the Table_infos outside duplicate mode and the
+    // final state outside single-table mode
+    static const char* names[26] = {"keys", "deal_table", "pool", "scratch", "cum_return", "acc", "sums", "status", BRL_TABLE_INFO_NAMES,
+                                    "final state", "observation", "mask", "rewards", "terminated", "current_player"};
+    const bool dup = mode == BRL_EVAL_MATCH_DUPLICATE, single = mode == BRL_EVAL_MATCH_SINGLE;
+    const uint8_t t16 = dup ? 16 : 0, f16 = single ? 16 : 0;
+    const uint8_t align[26] = {16, 16, 16, 16, 4, full ? 4 : 0, full ? 8 : 0, 4, 0, t16, 0, 0, 0, 0, 0, t16, 0, 0, 0, 0,
+                               f16, f16, single ? 2 : 0, f16, 0, 0};
+    const unsigned nullable = (full ? 0u : 1u << 5 | 1u << 6) | 0xFFFu << 8 | 0x3Fu << 20;
+    if ((rc = check_buffers("brl_evaluate_match", b, names, 26, nullable, 0u, align))) return rc;
+    const int tables = dup ? given(b, 8, 20) : 0, finals = single ? given(b, 20, 26) : 0;
+    if (tables != 0 && tables != 12) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all twelve Table_info buffers [8..19] or none");
+    if (finals != 0 && finals != 6) return fail(BRL_E_BUFFER, "brl_evaluate_match: give all six final-state buffers [20..25] or none");
 
     MatchPlan q = base_plan("brl_evaluate_match", mode, p, partner ? 3 : 2, b[3], partner);
     q.free_run = free_run;
@@ -936,10 +904,10 @@ int32_t brl_evaluate_match(brl_stream_t stream, void** b, const void* opaque, si
         q.sums = static_cast<double*>(b[6]);
         q.logits = q.at<float>(q.L.logits);
     }
-    if (mode == BRL_EVAL_MATCH_DUPLICATE && tables)
+    if (tables)
         for (int t = 0; t < 2; ++t)
             for (int k = 0; k < 6; ++k) q.info[t][k] = b[8 + 6 * t + k];
-    if (mode == BRL_EVAL_MATCH_SINGLE) {
+    if (single) {
         q.rewards_sum = q.at<float>(q.L.rewards_sum);
         if (finals) {
             q.state = b[20];
@@ -974,23 +942,17 @@ int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_
     if (p->n_deals <= 0) return fail(BRL_E_OPAQUE, "brl_call_values: n_deals must be > 0");
     if (p->flags & BRL_F_SAMPLE) return fail(BRL_E_OPAQUE, "brl_call_values: sampling is not supported (argmax only)");
     if (cap < 0) return fail(BRL_E_OPAQUE, "brl_call_values: the record capacity (seed) must be >= 0");
-    static const char* names[] = {"keys", "deal_table", "pool", "env_models", "rewards_a", "rewards_b", "scratch", "gain_sums",
-                                  "regret_sums", "mismatch", "status"};
-    if ((rc = check_buffers("brl_call_values", b, names, 11, 0u, 1u << 0 | 1u << 2 | 1u << 4 | 1u << 5 | 1u << 6)) != BRL_OK) return rc;
-    if (misaligned(b[3], 16) || misaligned(b[7], 8) || misaligned(b[8], 8) || misaligned(b[9], 8) || misaligned(b[10], 4))
-        return fail(BRL_E_BUFFER, "brl_call_values: env_models must be 16-byte, the sums 8-byte and status 4-byte aligned");
-    int given = 0;
-    for (int k = 11; k < 19; ++k) given += b[k] != nullptr;
-    if (given != 0 && given != 8) return fail(BRL_E_BUFFER, "brl_call_values: give all eight record buffers [11..18] or none");
-    if (given && (misaligned(b[11], 8) || misaligned(b[12], 4) || misaligned(b[13], 4) || misaligned(b[14], 4) ||
-                  misaligned(b[15], 4) || misaligned(b[16], 4) || misaligned(b[17], 4) || misaligned(b[18], 4)))
-        return fail(BRL_E_BUFFER, "brl_call_values: the record count must be 8-byte and the records 4-byte aligned");
+    static const char* names[21] = {"keys", "deal_table", "pool", "env_models", "rewards_a", "rewards_b", "scratch", "gain_sums",
+                                    "regret_sums", "mismatch", "status", "count", "env", "table", "player", "net", "context", "played",
+                                    "r", "obs", "gain"};
+    static const uint8_t align[21] = {16, 0, 16, 16, 16, 16, 16, 8, 8, 8, 4, 8, 4, 4, 4, 4, 4, 4, 4, 16, 4};
+    if ((rc = check_buffers("brl_call_values", b, names, 21, 0x3FFu << 11, 0u, align))) return rc;
+    const int records = given(b, 11, 19);
+    if (records != 0 && records != 8) return fail(BRL_E_BUFFER, "brl_call_values: give all eight record buffers [11..18] or none");
     const bool examples = b[19] != nullptr;
     if (examples != (b[20] != nullptr))
         return fail(BRL_E_BUFFER, "brl_call_values: give both training-example buffers [19] obs and [20] gain, or neither");
-    if (examples && !given) return fail(BRL_E_BUFFER, "brl_call_values: the training examples [19], [20] need the eight record buffers [11..18]");
-    if (examples && (misaligned(b[19], 16) || misaligned(b[20], 4)))
-        return fail(BRL_E_BUFFER, "brl_call_values: the example obs [19] must be 16-byte and gain [20] 4-byte aligned");
+    if (examples && !records) return fail(BRL_E_BUFFER, "brl_call_values: the training examples [19], [20] need the eight record buffers [11..18]");
 
     CvPlan c{};
     c.q = base_plan("brl_call_values", 0, p, M, b[6]);
@@ -1015,7 +977,7 @@ int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_
     c.o.status = c.q.status;
     c.o.cap = cap;
     c.o.env_offset = p->env_offset;
-    if (given) {
+    if (records) {
         c.o.count = static_cast<unsigned long long*>(b[11]);
         c.o.env = static_cast<int32_t*>(b[12]);
         c.o.table = static_cast<int32_t*>(b[13]);

@@ -208,12 +208,15 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     } while (0)
 
 // An op's buffer checks, in buffer order: b[k] must not be NULL unless bit k of `nullable` is set, and must be 16-byte
-// aligned when bit k of `aligned16` is set.  `what` names the op in the message.
-inline int32_t check_buffers(const char* what, void* const* b, const char* const* names, int n, unsigned nullable, unsigned aligned16) {
+// aligned when bit k of `aligned16` is set, else align[k]-byte aligned when `align` is given (0 or 1: any address).  `what`
+// names the op in the message.
+inline int32_t check_buffers(const char* what, void* const* b, const char* const* names, int n, unsigned nullable, unsigned aligned16,
+                             const uint8_t* align = nullptr) {
     for (int k = 0; k < n; ++k) {
         if (b[k] == nullptr && !((nullable >> k) & 1u)) return fail(BRL_E_BUFFER, "%s: buffer '%s' is NULL", what, names[k]);
-        if (((aligned16 >> k) & 1u) && (reinterpret_cast<uintptr_t>(b[k]) & 15u) != 0)
-            return fail(BRL_E_BUFFER, "%s: buffer '%s' is not 16-byte aligned", what, names[k]);
+        const unsigned a = (aligned16 >> k) & 1u ? 16u : align != nullptr && align[k] > 1 ? align[k] : 1u;
+        if ((reinterpret_cast<uintptr_t>(b[k]) & (a - 1)) != 0)
+            return fail(BRL_E_BUFFER, "%s: buffer '%s' is not %u-byte aligned", what, names[k], a);
     }
     return BRL_OK;
 }

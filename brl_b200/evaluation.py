@@ -58,12 +58,21 @@ def _bf16_state(env, keys):
     return State(env, packed, out)
 
 
+def _opponent_params(eval_env, team2_params, team2_model_path, game_mode: str = "competitive"):
+    """team 2's net: `team2_params`, else the pickle at `team2_model_path`; None in "free-run" (team 2 always passes)"""
+    if game_mode == "competitive":
+        return team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
+    if game_mode == "free-run":
+        return None
+    raise ValueError(game_mode)
+
+
 def make_simple_evaluate(eval_env, team1_activation, team1_model_type, team2_activation, team2_model_type,
                          team2_model_path, num_eval_envs, team2_params=None):
     """src/evaluation.py:11-66: deterministic quad steps vs a fixed opponent; mean raw score."""
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
-    opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
+    opp_params = _opponent_params(eval_env, team2_params, team2_model_path)
 
     def simple_evaluate(actor_params, rng, trace=None, partner_params=None):
         """`trace` (a list, tests only) receives the four sub-step action tensors of every quad step and finally
@@ -254,6 +263,44 @@ def _check_match_status(status: int, op: str = "brl_duplicate_match") -> None:
         raise ops._lib.BrlError(f"{op}: envs still live after {ops._lib.MATCH_MAX_STEPS} steps (status {status})")
 
 
+def _table_infos(tables):
+    """copies of a buffer set's two final TableInfoBuffers as Table_info"""
+    return [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
+                       t.call_xx.clone()) for t in tables]
+
+
+def _fill_chunk(b, board_keys, g, n: int, nets) -> None:
+    """keys and env_models of a chunk of global envs g: env g plays board g % n with the nets of match g // n"""
+    b.keys.copy_(board_keys[torch.as_tensor(g % n, device=b.keys.device)])
+    b.env_models.copy_(torch.as_tensor(nets[g // n], device=b.keys.device))
+
+
+def _play_single(eval_env, sets, new_set, partnered: bool, rng_key, env_offset: int, nets, play, op: str):
+    """One call of a single-match device evaluator: the buffer set of `sets` for the partner flag (allocated by
+    `new_set(partnered)` at its first use), the keys of the match (src/evaluation.py:93-94), nets = [(forward_pass, params)]
+    packed into pool slots 0 / 1 / 2 (None params: the slot is not read), `play(b)`, then one host copy of the all-reduced
+    sums (a copy: the buffers keep theirs) with the status, or of the status alone where the set has no sums; the status is
+    checked.  Returns (b, host sums or None)."""
+    if partnered not in sets:
+        sets[partnered] = new_set(partnered)
+    b = sets[partnered]
+    _, sub_key = brandom.split(rng_key)
+    b.keys.copy_(eval_env.make_keys(sub_key, b.keys.shape[0], env_offset))
+    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+    for slot, (forward_pass, params) in enumerate(nets):
+        if params is not None:
+            forward_pass.pack_into(params, b.pool[slot, :blob_bytes])
+    play(b)
+    if b.sums is None:
+        _check_match_status(int(b.status[0]), op)
+        return b, None
+    sums = b.sums.clone()
+    bdist.allreduce_sums(sums)
+    host = torch.cat((sums, b.status.to(torch.float64))).cpu()
+    _check_match_status(int(host[-1]), op)
+    return b, host[:-1]
+
+
 def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_envs, env_offset: int = 0, *, tune: int = 0):
     """make_simple_duplicate_evaluate (src/evaluation.py:69-204) with the whole match in one brl_duplicate_match call: the
     loop runs on the device (a CUDA graph WHILE node), so a match costs one launch and one host read of its statistics.
@@ -265,32 +312,23 @@ def make_device_duplicate_evaluate(eval_env, activation, model_type, num_eval_en
     player id, BRL_F_PLAYER_MODELS; its own buffers and graph)."""
     forward_pass = make_forward_pass(activation=activation, model_type=model_type)
     n, dev = num_eval_envs, eval_env.device
-    bufs = _MatchBuffers(n, 2, 0, dev, with_models=False, with_tables=True)
-    partner_bufs = []                                           # allocated at the first call with a partner
-    blob_bytes = ops._lib.load().brl_mlp_packed_bytes()
+    single_bf16 = forward_pass.precision == "tc-bf16"
+
+    def new_set(partnered):
+        if not partnered:
+            return _MatchBuffers(n, 2, 0, dev, with_models=False, with_tables=True)
+        b = _MatchBuffers(n, 3, 0, dev, with_models=True, with_tables=True, players=True)
+        b.env_models.copy_(torch.tensor([0, 2, 1, 1], dtype=torch.int32, device=dev).expand(n, 4))
+        return b
+
+    sets = {False: new_set(False)}                              # with a partner: a 3-net set, allocated at its first call
 
     def duplicate_evaluate(team1_params, team2_params, rng_key, team1_partner=None):
-        if team1_partner is not None:
-            if not partner_bufs:
-                partner_bufs.append(_MatchBuffers(n, 3, 0, dev, with_models=True, with_tables=True, players=True))
-                partner_bufs[0].env_models.copy_(torch.tensor([0, 2, 1, 1], dtype=torch.int32, device=dev).expand(n, 4))
-            b = partner_bufs[0]
-            forward_pass.pack_into(team1_partner, b.pool[2, :blob_bytes])
-        else:
-            b = bufs
-        rng_key, sub_key = brandom.split(rng_key)
-        b.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))                          # :93-94
-        forward_pass.pack_into(team1_params, b.pool[0, :blob_bytes])
-        forward_pass.pack_into(team2_params, b.pool[1, :blob_bytes])
-        b.play(eval_env, forward_pass.precision == "tc-bf16", tune)                         # :95-198
-        sums = b.sums.clone()
-        bdist.allreduce_sums(sums)
-        host = torch.cat((sums, b.status.to(torch.float64))).cpu()
-        _check_match_status(int(host[8]))
-        log_info = bdist.stats_from_sums(host[:8])                                        # :199-201
-        infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
-                            t.call_xx.clone()) for t in b.tables]
-        return log_info, infos[0], infos[1], b.cum_return.clone()
+        b, sums = _play_single(eval_env, sets, new_set, team1_partner is not None, rng_key, env_offset,
+                               [(forward_pass, team1_params), (forward_pass, team2_params), (forward_pass, team1_partner)],
+                               lambda b: b.play(eval_env, single_bf16, tune), "brl_duplicate_match")     # :93-198
+        infos = _table_infos(b.tables)
+        return bdist.stats_from_sums(sums), infos[0], infos[1], b.cum_return.clone()    # :199-201
 
     return duplicate_evaluate
 
@@ -389,8 +427,7 @@ def _make_device_pair_matches(eval_env, forward_pass, num_eval_envs: int, max_en
                     b = buffers[key]
                     for m, params in enumerate(params_list):
                         forward_pass.pack_into(params, b.pool[m, :blob_bytes])
-                b.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
-                b.env_models.copy_(torch.as_tensor(pair_arr[c0 + g // n], device=dev))
+                _fill_chunk(b, board_keys, g, n, pair_arr[c0:])
                 b.offsets.copy_(torch.as_tensor(bounds, device=dev))
                 if system_hist is None:
                     b.play(eval_env, single_bf16, tune)
@@ -579,8 +616,7 @@ def make_call_values_evaluate(eval_env, activation, model_type, num_eval_envs: i
             for m, params in enumerate(params_list):
                 forward_pass.pack_into(params, b.match.pool[m, :blob_bytes])
             g = np.arange(c0, c1)
-            b.match.keys.copy_(board_keys[torch.as_tensor(g % n, device=dev)])
-            b.match.env_models.copy_(torch.as_tensor(pairs[g // n], device=dev))
+            _fill_chunk(b.match, board_keys, g, n, pairs)
             b.match.play(eval_env, single_bf16, tune)
             if records and (b.records is None or b.records.train != train):
                 b.records = ops.CallValueRecords(48 * (c1 - c0), dev, train)  # about twice a typical board's decisions
@@ -698,12 +734,7 @@ def make_evaluate(eval_env, team1_activation, team1_model_type, team2_activation
     actor's architecture) instead of the actor, which then plays player 0 only."""
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
-    if game_mode == "competitive":
-        opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
-    elif game_mode == "free-run":
-        opp_params = None
-    else:
-        raise ValueError(game_mode)
+    opp_params = _opponent_params(eval_env, team2_params, team2_model_path, game_mode)
     n, dev = num_eval_envs, eval_env.device
     n_sums = ops._lib.load().brl_eval_num_sums()
 
@@ -844,36 +875,19 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
     L = ops._lib
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
-    if game_mode == "competitive":
-        opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
-    elif game_mode == "free-run":
-        opp_params = None
-    else:
-        raise ValueError(game_mode)
+    opp_params = _opponent_params(eval_env, team2_params, team2_model_path, game_mode)
     single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
     n, dev = num_eval_envs, eval_env.device
     mode = L.EVAL_MATCH_DUPLICATE if duplicate else L.EVAL_MATCH_SINGLE
     sets = {False: _EvalBuffers(n, mode, dev)}                  # with a partner: a 3-net set, allocated at its first call
-    blob_bytes = L.load().brl_mlp_packed_bytes()
 
     def play(actor_params, rng_key, partner_params):
-        partnered = partner_params is not None
-        if partnered not in sets:
-            sets[partnered] = _EvalBuffers(n, mode, dev, partner=True)
-        fn.buffers = bufs = sets[partnered]
-        rng_key, sub_key = brandom.split(rng_key)
-        bufs.keys.copy_(eval_env.make_keys(sub_key, n, env_offset))
-        actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
-        if opp_params is not None:
-            opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
-        if partnered:
-            actor_forward_pass.pack_into(partner_params, bufs.pool[2, :blob_bytes])
-        bufs.play(eval_env, single_bf16, opp_params is None, tune)
-        sums = bufs.sums.clone()
-        bdist.allreduce_sums(sums)
-        host = torch.cat((sums, bufs.status.to(torch.float64))).cpu().numpy()
-        _check_match_status(int(host[-1]), "brl_evaluate_match")
-        return host[:-1]
+        fn.buffers, sums = _play_single(
+            eval_env, sets, lambda partnered: _EvalBuffers(n, mode, dev, partner=partnered), partner_params is not None,
+            rng_key, env_offset,
+            [(actor_forward_pass, actor_params), (opp_forward_pass, opp_params), (actor_forward_pass, partner_params)],
+            lambda b: b.play(eval_env, single_bf16, opp_params is None, tune), "brl_evaluate_match")
+        return sums.numpy()
 
     def evaluate(actor_params, rng_key, partner_params=None):
         sums = play(actor_params, rng_key, partner_params)
@@ -885,8 +899,7 @@ def make_device_evaluate(eval_env, team1_activation, team1_model_type, team2_act
 
     def duplicate_evaluate(actor_params, rng_key, partner_params=None):
         sums = play(actor_params, rng_key, partner_params)
-        infos = [Table_info(t.terminated.clone(), t.rewards.clone(), t.last_bid.clone(), t.last_bidder.clone(), t.call_x.clone(),
-                            t.call_xx.clone()) for t in fn.buffers.tables]
+        infos = _table_infos(fn.buffers.tables)
         return _log_info_from_sums(sums, duplicate=True), infos[0], infos[1]
 
     fn = duplicate_evaluate if duplicate else evaluate
@@ -922,25 +935,20 @@ def make_device_simple_evaluate(eval_env, team1_activation, team1_model_type, te
     L = ops._lib
     actor_forward_pass = make_forward_pass(activation=team1_activation, model_type=team1_model_type)
     opp_forward_pass = make_forward_pass(activation=team2_activation, model_type=team2_model_type)
-    opp_params = team2_params if team2_params is not None else load_params(team2_model_path, eval_env.device)
+    opp_params = _opponent_params(eval_env, team2_params, team2_model_path)
     single_bf16 = _one_precision(actor_forward_pass, opp_forward_pass)
-    sets = {False: _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device)}
-    blob_bytes = L.load().brl_mlp_packed_bytes()
+
+    def new_set(partnered):
+        return _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device, partner=partnered)
+
+    sets = {False: new_set(False)}
 
     def simple_evaluate(actor_params, rng, partner_params=None):
-        partnered = partner_params is not None
-        if partnered not in sets:
-            sets[partnered] = _EvalBuffers(num_eval_envs, L.EVAL_MATCH_SIMPLE, eval_env.device, partner=True)
-        simple_evaluate.buffers = bufs = sets[partnered]
-        rng_key, sub_key = brandom.split(rng)
-        bufs.keys.copy_(eval_env.make_keys(sub_key, num_eval_envs))
-        actor_forward_pass.pack_into(actor_params, bufs.pool[0, :blob_bytes])
-        opp_forward_pass.pack_into(opp_params, bufs.pool[1, :blob_bytes])
-        if partnered:
-            actor_forward_pass.pack_into(partner_params, bufs.pool[2, :blob_bytes])
-        bufs.play(eval_env, single_bf16, False, tune)
-        _check_match_status(int(bufs.status[0]), "brl_evaluate_match")
-        return bufs.cum_return.mean()
+        simple_evaluate.buffers, _ = _play_single(
+            eval_env, sets, new_set, partner_params is not None, rng, 0,
+            [(actor_forward_pass, actor_params), (opp_forward_pass, opp_params), (actor_forward_pass, partner_params)],
+            lambda b: b.play(eval_env, single_bf16, False, tune), "brl_evaluate_match")
+        return simple_evaluate.buffers.cum_return.mean()
 
     simple_evaluate.buffers = sets[False]
     return simple_evaluate

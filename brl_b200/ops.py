@@ -712,6 +712,24 @@ def mlp_pack_pool(params_list, pack_one) -> torch.Tensor:
     return pool
 
 
+def _check_pool(who: str, pool: torch.Tensor, n_nets: Optional[int] = None, min_nets: int = 0, suffix: str = "") -> None:
+    """pool u8[M, mlp_pool_stride()], with M = n_nets when given and M >= min_nets"""
+    if pool.dim() != 2 or pool.dtype != torch.uint8 or pool.shape[1] != mlp_pool_stride() or pool.shape[0] < min_nets or \
+            (n_nets is not None and pool.shape[0] != n_nets):
+        raise _lib.BrlError(f"{who}: pool must be u8[{'M' if n_nets is None else n_nets}, mlp_pool_stride()] (ops.mlp_pack_pool)"
+                            + suffix)
+
+
+def _check_env_models(who: str, env_models: torch.Tensor, n: int) -> None:
+    if env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4)):
+        raise _lib.BrlError(f"{who}: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+
+
+def _check_deal_table(who: str, table: torch.Tensor) -> None:
+    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
+        raise _lib.BrlError(f"{who}: the deal table must be u8 [n_deals, 48]")
+
+
 def model_rows(current_player: torch.Tensor, done: Optional[torch.Tensor], env_models: torch.Tensor, rows: torch.Tensor,
                counts: torch.Tensor, offsets: torch.Tensor, block_model: torch.Tensor) -> None:
     """Live envs (done == 0) grouped by the net that acts there: env_models[i, 0] for players 0/1, [i, 1] for players 2/3,
@@ -719,9 +737,7 @@ def model_rows(current_player: torch.Tensor, done: Optional[torch.Tensor], env_m
     row count and block_model the net of each 256-row block.  A live env whose id is outside [0, M) makes offsets[M] = -1:
     the grouping is invalid, and the caller's read of offsets[M] (which sizes the forward) must raise."""
     n_models = counts.shape[0]
-    if env_models.dtype != torch.int32 or env_models.dim() != 2 or tuple(env_models.shape) not in \
-            ((current_player.shape[0], 2), (current_player.shape[0], 4)):
-        raise _lib.BrlError("model_rows: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    _check_env_models("model_rows", env_models, current_player.shape[0])
     if offsets.shape[0] != n_models + 1 or rows.shape[0] < model_rows_capacity(current_player.shape[0], n_models):
         raise _lib.BrlError("model_rows: offsets must hold M + 1 entries and rows model_rows_capacity(n, M)")
     flags = _lib.F_PLAYER_MODELS if env_models.shape[1] == 4 else 0
@@ -747,8 +763,7 @@ def policy_act_grouped(obs_bf16: torch.Tensor, pool: torch.Tensor, scratch: torc
         n_rows = torch.full((1,), n, dtype=torch.int32, device=rows.device)
     if not n_rows.is_cuda or n_rows.dtype != torch.int32 or n_rows.numel() < 1:
         raise _lib.BrlError("policy_act_grouped: n_rows must be a CUDA int32 tensor holding the padded row count (offsets[M:])")
-    if pool.dim() != 2 or pool.shape[1] != mlp_pool_stride() or pool.dtype != torch.uint8:
-        raise _lib.BrlError("policy_act_grouped: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    _check_pool("policy_act_grouped", pool)
     if scratch.numel() < _lib.load().brl_mlp_rows_scratch_bytes(n):
         raise _lib.BrlError("policy_act_grouped: scratch too small (ops.policy_grouped_scratch_bytes)")
     _call("brl_policy_act_grouped", [_ptr(obs_bf16), _ptr(pool), _ptr(scratch), _ptr(mask), _ptr(action), _ptr(rows),
@@ -792,8 +807,8 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
     n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
     if env_models is None and M != 2:
         raise _lib.BrlError(f"duplicate_match: without env_models the pool must hold 2 nets, got {M}")
-    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4))):
-        raise _lib.BrlError("duplicate_match: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    if env_models is not None:
+        _check_env_models("duplicate_match", env_models, n)
     player_models = env_models is not None and env_models.shape[1] == 4
     P = 0
     if range_offsets is not None:
@@ -804,8 +819,7 @@ def duplicate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor,
         raise _lib.BrlError("duplicate_match: without range_offsets sums is float64[8]")
     if sums.dtype != torch.float64 or cum_return.dtype != torch.float32 or status.dtype != torch.int32:
         raise _lib.BrlError("duplicate_match: sums must be float64, cum_return float32 and status int32")
-    if pool.dim() != 2 or pool.dtype != torch.uint8 or pool.shape[1] != mlp_pool_stride():
-        raise _lib.BrlError("duplicate_match: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
+    _check_pool("duplicate_match", pool)
     if scratch.numel() < duplicate_match_scratch_bytes(n, M):
         raise _lib.BrlError("duplicate_match: scratch too small (ops.duplicate_match_scratch_bytes)")
     if (table_a is None) != (table_b is None):
@@ -850,10 +864,7 @@ def evaluate_match(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, 
     full = mode != _lib.EVAL_MATCH_SIMPLE
     if free_run and not full:
         raise _lib.BrlError("evaluate_match: free_run is a mode of the full-statistics evaluation")
-    n_nets = 3 if partner else 2
-    if pool.dim() != 2 or pool.dtype != torch.uint8 or tuple(pool.shape) != (n_nets, mlp_pool_stride()):
-        raise _lib.BrlError(f"evaluate_match: pool must be u8[{n_nets}, mlp_pool_stride()] (ops.mlp_pack_pool)"
-                            + (" with the partner's net" if partner else ""))
+    _check_pool("evaluate_match", pool, 3 if partner else 2, suffix=" with the partner's net" if partner else "")
     if cum_return.dtype != torch.float32 or status.dtype != torch.int32:
         raise _lib.BrlError("evaluate_match: cum_return must be float32 and status int32")
     if full:
@@ -913,10 +924,9 @@ def system_stats(state: torch.Tensor, table: torch.Tensor, action: torch.Tensor,
         raise _lib.BrlError("system_stats: action must be int32 [n]")
     if done is not None and (done.dtype not in (torch.uint8, torch.bool) or tuple(done.shape) != (n,)):
         raise _lib.BrlError("system_stats: done must be uint8 / bool [n]")
-    if env_models is not None and (env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4))):
-        raise _lib.BrlError("system_stats: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
-    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
-        raise _lib.BrlError("system_stats: the deal table must be u8 [n_deals, 48]")
+    if env_models is not None:
+        _check_env_models("system_stats", env_models, n)
+    _check_deal_table("system_stats", table)
     flags = _lib.F_PLAYER_MODELS if env_models is not None and env_models.shape[1] == 4 else 0
     _call("brl_system_stats", [_ptr(state), _ptr(table), _ptr(action), _ptr(done), _ptr(env_models), _ptr(hist)],
           _params(n, stride=state.shape[1], k_steps=M, n_deals=table.shape[0], flags=flags))
@@ -933,8 +943,7 @@ def system_stats_auctions(table: torch.Tensor, calls: torch.Tensor, offsets: tor
         raise _lib.BrlError("system_stats_auctions: offsets must be int64 [n + 1]")
     if calls.dtype != torch.uint8 or calls.dim() != 1:
         raise _lib.BrlError("system_stats_auctions: calls must be u8 [total]")
-    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
-        raise _lib.BrlError("system_stats_auctions: the deal table must be u8 [n_deals, 48]")
+    _check_deal_table("system_stats_auctions", table)
     if board is not None and (board.dtype != torch.int32 or tuple(board.shape) != (n,)):
         raise _lib.BrlError("system_stats_auctions: board must be int32 [n]")
     if dealer is not None and (dealer.dtype != torch.int8 or tuple(dealer.shape) != (n,)):
@@ -1003,15 +1012,12 @@ def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env
     n, M = int(keys.shape[0]), int(pool.shape[0]) if pool.dim() == 2 else 0
     if keys.dtype != torch.int64 or keys.dim() != 1:
         raise _lib.BrlError("call_values: keys must be int64 [n] (ops.make_keys)")
-    if pool.dim() != 2 or pool.dtype != torch.uint8 or pool.shape[1] != mlp_pool_stride() or M < 1:
-        raise _lib.BrlError("call_values: pool must be u8[M, mlp_pool_stride()] (ops.mlp_pack_pool)")
-    if env_models.dtype != torch.int32 or tuple(env_models.shape) not in ((n, 2), (n, 4)):
-        raise _lib.BrlError("call_values: env_models must be int32 [n, 2] (by team) or [n, 4] (by player)")
+    _check_pool("call_values", pool, min_nets=1)
+    _check_env_models("call_values", env_models, n)
     for name, t in (("rewards_a", rewards_a), ("rewards_b", rewards_b)):
         if t.dtype != torch.float32 or tuple(t.shape) != (n, 4):
             raise _lib.BrlError(f"call_values: {name} must be float32 [n, 4] (a Table_info's rewards)")
-    if table.dtype != torch.uint8 or table.dim() != 2 or table.shape[1] != 48:
-        raise _lib.BrlError("call_values: the deal table must be u8 [n_deals, 48]")
+    _check_deal_table("call_values", table)
     if gain_sums.dtype != torch.int64 or tuple(gain_sums.shape) != (M,) + CALL_GAIN_SHAPE:
         raise _lib.BrlError(f"call_values: gain_sums must be int64 [{M}, 75, 38, 38, 4]")
     if regret_sums.dtype != torch.int64 or tuple(regret_sums.shape) != (M,) + CALL_REGRET_SHAPE:

@@ -8,9 +8,9 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the loss-head refactor (the warp reductions, the dz store, the selected softmax and the block-sum
-tail of k_ppo_loss, k_sl_loss and k_cv_loss moved into csrc/loss_head.cuh): no kernel is renamed, added or removed.
-Replace both tables for another change."""
+RENAMES and ADDED record the match-op refactor of csrc/brl_match.cu: brl_call_values' control kernel k_cv_control (a bound
+parameter and a stop once a loop has failed) is now the one control kernel of all three ops, under the name k_match_control,
+and the old k_match_control is removed.  Nothing is added.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -18,7 +18,8 @@ import subprocess
 import sys
 from collections import OrderedDict
 
-RENAMES = []  # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
+# (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
+RENAMES = [(r"^brl::k_match_control$", None), (r"^brl::k_cv_control$", "brl::k_match_control")]
 ADDED = []  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
