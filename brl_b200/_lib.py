@@ -17,7 +17,8 @@ from . import build as _build
 LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "brl_policy_act_grouped", "brl_match_stats_ranges",
             "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped",
             "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats",
-            "brl_system_stats", "brl_system_stats_auctions", "brl_call_values", "brl_cv_grad", "brl_cv_eval")
+            "brl_system_stats", "brl_system_stats_auctions", "brl_call_values", "brl_cv_grad", "brl_cv_eval",
+            "brl_hand_posterior")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -35,7 +36,8 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_mlp_pool_stride", "brl_model_rows_capacity", "brl_policy_grouped_scratch_bytes",
         "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes",
         "brl_evaluate_match_partner_scratch_bytes",
-        "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride", "brl_call_values_scratch_bytes")
+        "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride", "brl_call_values_scratch_bytes",
+        "brl_hand_posterior_scratch_bytes")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 
@@ -65,6 +67,10 @@ F_EVAL_FREE_RUN = 0x0008  # brl_evaluate_match: team 2 always passes (BRL_F_EVAL
 F_EVAL_PARTNER = 1 << 25  # brl_evaluate_match: a 3-net pool, net 2 the actor's partner (BRL_F_EVAL_PARTNER)
 F_PLAYER_MODELS = 1 << 24  # brl_model_rows / brl_duplicate_match: env_models[n, 4] by player id (BRL_F_PLAYER_MODELS)
 SYS_CONTEXTS, SYS_COLS = 75, 96  # the bidding-system histogram hist[M, 75, 38, 96] (BRL_SYS_*)
+# brl_hand_posterior's per-query status codes (BRL_POST_*) and its Philox stream tag
+POST_OK, POST_ILLEGAL, POST_SHORT, POST_BAD_NET, POST_BAD_QUERY, POST_CAPACITY = 0, 1, 2, 3, 4, 5
+POST_TAG = 0x484E4430
+POST_FEATURES = 95
 
 
 def f_eval_match(mode: int) -> int:

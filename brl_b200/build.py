@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libbrl_b200.so")
-SOURCES = ["brl_env.cu", "brl_algo.cu", "brl_mlp.cu", "brl_mlp_train.cu", "brl_ppo.cu", "brl_eval.cu", "brl_sl.cu", "brl_cv.cu", "brl_match.cu", "brl_host.cu", "xla_ffi_shim.cc"]
+SOURCES = ["brl_env.cu", "brl_algo.cu", "brl_mlp.cu", "brl_mlp_train.cu", "brl_ppo.cu", "brl_eval.cu", "brl_sl.cu", "brl_cv.cu", "brl_match.cu", "brl_posterior.cu", "brl_host.cu", "xla_ffi_shim.cc"]
 NVCC_FLAGS = [
     "-std=c++17", "-O3", "-lineinfo",
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -88,6 +88,7 @@
     X(brl_call_values, "iiiiiisoooooooooooo") \
     X(brl_cv_grad, "iisioos") \
     X(brl_cv_eval, "iisios") \
+    X(brl_hand_posterior, "iiiiiiiiisoooo") \
     /* end */
 
 namespace {

@@ -1039,3 +1039,78 @@ def call_values(keys: torch.Tensor, table: torch.Tensor, pool: torch.Tensor, env
           _params(n, k_steps=M, n_deals=table.shape[0], flags=flags, env_offset=env_offset,
                   seed=records.capacity if records is not None else 0, illegal_penalty=illegal_penalty,
                   illegal_bonus=illegal_bonus))
+
+
+# ---- hand reading (DESIGN.md f18) -------------------------------------------------------------------------------------------
+def hand_posterior_scratch_bytes(n_queries: int, n_samples: int, row_capacity: int, n_models: int) -> int:
+    return _size_query("brl_hand_posterior_scratch_bytes", n_queries, n_samples, row_capacity, n_models)
+
+
+def hand_posterior(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tensor, query: torch.Tensor, seat_nets: torch.Tensor,
+                   pool: torch.Tensor, scratch: torch.Tensor, cards: torch.Tensor, features: torch.Tensor, weights: torch.Tensor,
+                   status: torch.Tensor, *, samples: int, row_capacity: int, board: Optional[torch.Tensor] = None,
+                   dealer: Optional[torch.Tensor] = None, vul: Optional[torch.Tensor] = None, seed: int = 0, query_offset: int = 0,
+                   temperature: float = 1.0, single_bf16: bool = False, path_flags: int = 0, hands: Optional[torch.Tensor] = None,
+                   logw: Optional[torch.Tensor] = None) -> None:
+    """The posterior of the hidden hands for Q queries (brl_hand_posterior, DESIGN.md f18): query[j] = (t, s, L) reads the first L
+    calls of auction t (calls[offsets[t]:offsets[t + 1]], u8 0..37, on deal row board[t] (None: row t), dealer dealer[t] (int8;
+    None: North), vulnerability vul[t] (u8, bit 0 NS, bit 1 EW; None: none)) from absolute seat s, with net seat_nets[j, seat]
+    (int32 [Q, 4]) of `pool` at each seat.  Writes cards f64[Q, 3, 52], features f64[Q, 3, 95], weights f64[Q, 4] and status
+    int32[Q]; hands u64 (int64) [Q, N, 4] and logw f64[Q, N] are optional diagnostics, both or neither.  `row_capacity` (a
+    multiple of 256) sizes the forward; the scratch is hand_posterior_scratch_bytes(Q, N, row_capacity, M) bytes.  Every
+    argument is checked on the host (one device-to-host copy of offsets, calls and query) before any device work."""
+    who = "hand_posterior"
+    n = int(offsets.shape[0]) - 1 if offsets.dim() == 1 else -1
+    Q = int(query.shape[0]) if query.dim() == 2 else -1
+    N = int(samples)
+    if offsets.dtype != torch.int64 or n < 0:
+        raise _lib.BrlError(f"{who}: offsets must be int64 [n + 1]")
+    if calls.dtype != torch.uint8 or calls.dim() != 1:
+        raise _lib.BrlError(f"{who}: calls must be u8 [total]")
+    _check_deal_table(who, table)
+    for name, t, dt in (("board", board, torch.int32), ("dealer", dealer, torch.int8), ("vul", vul, torch.uint8)):
+        if t is not None and (t.dtype != dt or tuple(t.shape) != (n,)):
+            raise _lib.BrlError(f"{who}: {name} must be {str(dt).replace('torch.', '')} [n]")
+    if query.dtype != torch.int32 or tuple(query.shape) != (Q, 3):
+        raise _lib.BrlError(f"{who}: query must be int32 [Q, 3] = (auction, observer seat, prefix length)")
+    if seat_nets.dtype != torch.int32 or tuple(seat_nets.shape) != (Q, 4):
+        raise _lib.BrlError(f"{who}: seat_nets must be int32 [Q, 4]")
+    _check_pool(who, pool)
+    M = int(pool.shape[0])
+    if not 1 <= N <= 1 << 24:
+        raise _lib.BrlError(f"{who}: samples must be in [1, 2^24]")
+    if row_capacity < 0 or row_capacity % 256 or row_capacity > 1 << 30:
+        raise _lib.BrlError(f"{who}: row_capacity must be a multiple of 256 in [0, 2^30]")
+    if not (temperature >= 0.0) or temperature == float("inf"):
+        raise _lib.BrlError(f"{who}: temperature must be finite and >= 0")
+    if path_flags & ~(_lib.F_TUNE_MLP_LAYERS | _lib.F_TUNE_MLP_FUSED):
+        raise _lib.BrlError(f"{who}: path_flags may hold F_TUNE_MLP_LAYERS / F_TUNE_MLP_FUSED only")
+    for name, t, shape, dt in (("cards", cards, (Q, 3, 52), torch.float64), ("features", features, (Q, 3, _lib.POST_FEATURES), torch.float64),
+                               ("weights", weights, (Q, 4), torch.float64), ("status", status, (Q,), torch.int32)):
+        if t.dtype != dt or tuple(t.shape) != shape:
+            raise _lib.BrlError(f"{who}: {name} must be {str(dt).replace('torch.', '')} {list(shape)}")
+    if (hands is None) != (logw is None):
+        raise _lib.BrlError(f"{who}: hands and logw go together")
+    if hands is not None and (hands.dtype != torch.int64 or tuple(hands.shape) != (Q, N, 4) or logw.dtype != torch.float64
+                              or tuple(logw.shape) != (Q, N)):
+        raise _lib.BrlError(f"{who}: hands must be int64 [Q, N, 4] and logw float64 [Q, N]")
+    if Q == 0:
+        return
+    need = hand_posterior_scratch_bytes(Q, N, row_capacity, M)
+    if scratch.dtype != torch.uint8 or scratch.dim() != 1 or scratch.numel() < need:
+        raise _lib.BrlError(f"{who}: scratch must be u8 [>= {need}] (hand_posterior_scratch_bytes)")
+    off, q, c = offsets.cpu(), query.cpu(), calls.cpu()
+    if int(off[0]) != 0 or bool((off[1:] < off[:-1]).any()) or int(off[-1]) != calls.shape[0]:
+        raise _lib.BrlError(f"{who}: offsets must rise from 0 to len(calls)")
+    if c.numel() and int(c.max()) >= NUM_ACTIONS:
+        raise _lib.BrlError(f"{who}: a call is outside 0..37")
+    if int(q[:, 0].min()) < 0 or int(q[:, 0].max()) >= n:
+        raise _lib.BrlError(f"{who}: a query's auction is outside [0, {n})")
+    if board is None and n > table.shape[0]:
+        raise _lib.BrlError(f"{who}: without board auction t needs deal row t: the table is too short")
+    flags = (F_MLP_BF16 if single_bf16 else 0) | int(path_flags)
+    _call("brl_hand_posterior",
+          [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(board), _ptr(dealer), _ptr(vul), _ptr(query), _ptr(seat_nets), _ptr(pool),
+           _ptr(scratch), _ptr(cards), _ptr(features), _ptr(weights), _ptr(status), _ptr(hands), _ptr(logw)],
+          BrlParams(Q, int(query_offset), int(row_capacity), int(seed) & 0xFFFFFFFFFFFFFFFF, int(table.shape[0]), flags, N, M,
+                    -1.0, 1.0, float(temperature), 0.0))  # BrlParams directly: _params would turn a capacity of 0 into Q

@@ -64,6 +64,8 @@
  *                         optionally each decision's observation and gains as training examples (DESIGN.md f17)
  *   brl_cv_grad / brl_cv_eval   not in the reference: the all-actions policy-gradient loss head on those examples, on the
  *                         tensor-core forward / backward of brl_sl_grad (DESIGN.md f17)
+ *   brl_hand_posterior    not in the reference: the hidden hands an auction implies under the nets' policies, by importance
+ *                         sampling of the unseen cards with the grouped forward as the likelihood (DESIGN.md f18)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -498,6 +500,55 @@ int32_t brl_system_stats_auctions(brl_stream_t, void **buffers, const void *opaq
 int64_t brl_call_values_scratch_bytes(int64_t n_envs, int64_t n_models);
 int32_t brl_call_values(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- hand reading (not in the reference; DESIGN.md f18, restated by tests/posterior_ref.py) -----------------------------
+ * What an observer can infer about the three hidden hands from an auction, under the nets' own policies.
+ * Auctions use brl_system_stats_auctions' encoding: auction t is calls[offsets[t], offsets[t + 1]) (calls 0..37) on deal row
+ * board[t] (NULL: row t) with dealer dealer[t] (NULL: North) and vulnerability vul[t] (bit 0 NS, bit 1 EW; NULL: none); call k
+ * is made by seat (dealer + k) mod 4.  Query j = query[j] = (t, s, L): auction t, the observer's absolute seat s, the prefix
+ * length L (0 <= L <= the auction's length).  seat_nets[j, 0..3] = the net of each absolute seat, an index into a pool of M
+ * packed nets brl_mlp_pool_stride() bytes apart.
+ *   Sample i of query j (global index g = env_offset + j): the 39 cards outside the observer's hand, in increasing card index
+ *   h[0..38], are shuffled by Fisher-Yates: for t = 0..37, with n = 38 - t, swap h[n] and h[mulhi(u_t, n + 1)], where u_t is
+ *   word (t mod 4) (x, y, z, w) of philox4x32(counter (g_lo, g_hi, BRL_POST_TAG + t / 4, i), key (seed_lo, seed_hi)).  Then
+ *   h[0..12] are the observer's left-hand opponent's (seat s + 1), h[13..25] partner's (s + 2), h[26..38] the right-hand
+ *   opponent's (s + 3).  The samples depend on (seed, g, i) only.
+ *   Likelihood: for every k < L whose caller sigma_k != s, o is sigma_k's observation after c_0 .. c_{k-1} (vulnerability and
+ *   history relative to sigma_k, sigma_k's hand from the sample), m its legal mask, l the logits of net seat_nets[j, sigma_k]
+ *   on o (bf16 observation, the grouped forward).  l_k = log softmax over the legal calls of l / tau at c_k, in f32 as
+ *   brl_categorical forms log_prob (x - max - log sum exp); with tau = 0, l_k = 0 when c_k is the masked argmax (first maximum)
+ *   and -inf otherwise.  log w[j, i] = sum of l_k in f64, k increasing.
+ *   Posterior (self-normalised importance weights under the uniform prior): M_j = max_i log w, w' = exp(log w - M_j),
+ *   W = sum w'.  cards[j, r, c] = sum w' [card c held by relative seat r] / W (r = 0 LHO, 1 partner, 2 RHO);
+ *   features[j, r, 0..94] = the w'-weighted distribution of that hand's features in brl_system_stats' columns (HCP 0..37,
+ *   38 + 14 suit + length, 94 balanced) / W; weights[j] = {M_j, W, sum w'^2, #(w > 0)} (ESS = W^2 / sum w'^2).  Every sum is f64
+ *   over i increasing, so the outputs are bit-identical across runs, chunkings and batch compositions.  A query without an
+ *   accepted sample, or with a status other than BRL_POST_OK, has NaN cards / features / weights[0..2] and a count of 0.
+ * The call: a check pass (one thread per (query, k)), the row layout (segment (j, k) = N consecutive rows, one per sample, in
+ * its net's group; groups padded to 256 rows, the padded count in device memory), the public pass (each segment's rotated
+ * history words, vulnerability bits, legal mask and call), the sampler, the observation expansion (bf16 rows, only the hand
+ * bits vary in a segment), the grouped forward of brl_policy_act_grouped with logits out (its path by brl_policy_act's rule on
+ * the row capacity: pass the exact padded row count to run the path of that count), the per-sample log-likelihood and a
+ * per-query reduction.  No host synchronisation; capturable.
+ * buffers: [0] in deal_table  [1] in u8 calls[]  [2] in i64 offsets[]  [3] in i32 board[] (NULL: row t)  [4] in i8 dealer[]
+ *          (NULL: North)  [5] in u8 vul[] (NULL: none)  [6] in i32 query[Q, 3]  [7] in i32 seat_nets[Q, 4]
+ *          [8] in pool u8[M, brl_mlp_pool_stride()]  [9] scratch (brl_hand_posterior_scratch_bytes(Q, N, capacity, M))
+ *          [10] out f64 cards[Q, 3, 52]  [11] out f64 features[Q, 3, 95]  [12] out f64 weights[Q, 4]  [13] out i32 status[Q]
+ *          [14] out u64 hands[Q, N, 4] by absolute seat  [15] out f64 logw[Q, N] -- diagnostics, both or neither
+ * params: n_envs = Q, env_offset = the global index of query 0, seed, step = N (samples per query, 1 .. 2^24), k_steps = M,
+ *         state_stride = the row capacity (a multiple of 256), n_deals = rows in the deal table, gamma = tau (>= 0; < 0 or NaN
+ *         is BRL_E_OPAQUE), flags BRL_F_MLP_BF16 | BRL_F_TUNE_MLP_LAYERS / BRL_F_TUNE_MLP_FUSED.  t must name an auction of the
+ *         buffers and calls must be in 0..37: they are not checked here.  An empty batch is a no-op. */
+#define BRL_POST_TAG 0x484E4430u  /* "HND0": Philox stream of the hand sampler, + block index 0..9 */
+#define BRL_POST_OK 0
+#define BRL_POST_ILLEGAL 1        /* a call of the prefix is not legal where it is made */
+#define BRL_POST_SHORT 2          /* the auction ends before call L, or L is longer than the auction */
+#define BRL_POST_BAD_NET 3        /* a seat that calls in the prefix (not the observer) has a net id outside [0, M) */
+#define BRL_POST_BAD_QUERY 4      /* s outside 0..3, L < 0, or the deal row outside the table */
+#define BRL_POST_CAPACITY 5       /* the layout needs more rows than the capacity: every query of the call, outputs invalid */
+#define BRL_POST_FEATURES 95
+int64_t brl_hand_posterior_scratch_bytes(int64_t n_queries, int64_t n_samples, int64_t row_capacity, int64_t n_models);
+int32_t brl_hand_posterior(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -787,6 +838,7 @@ void brl_call_values_xla(brl_stream_t, void **buffers, const char *opaque, size_
 void brl_cv_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_cv_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_hand_posterior_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------
  * Host-buffer convenience layer (the call a non-JAX host makes): the library

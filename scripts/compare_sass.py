@@ -8,9 +8,8 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the match-op refactor of csrc/brl_match.cu: brl_call_values' control kernel k_cv_control (a bound
-parameter and a stop once a loop has failed) is now the one control kernel of all three ops, under the name k_match_control,
-and the old k_match_control is removed.  Nothing is added.  Replace both tables for another change."""
+RENAMES and ADDED record the hand-reading change (DESIGN.md f18): no kernel is renamed or removed, and the kernels of
+csrc/brl_posterior.cu (brl::k_post_*) are added.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -19,8 +18,8 @@ import sys
 from collections import OrderedDict
 
 # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-RENAMES = [(r"^brl::k_match_control$", None), (r"^brl::k_cv_control$", "brl::k_match_control")]
-ADDED = []  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
+RENAMES = []
+ADDED = [r"^brl::k_post_"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):
