@@ -18,7 +18,7 @@ LAZY_OPS = ("brl_sl_examples", "brl_sl_grad", "brl_sl_eval", "brl_model_rows", "
             "brl_duplicate_match", "brl_evaluate_match", "brl_ppo_grad_grouped", "brl_mlp_adam_step_grouped",
             "brl_ppo_grad_anchored", "brl_ppo_grad_grouped_anchored", "brl_par", "brl_gather_reward_par", "brl_par_stats",
             "brl_system_stats", "brl_system_stats_auctions", "brl_call_values", "brl_cv_grad", "brl_cv_eval",
-            "brl_hand_posterior")
+            "brl_hand_posterior", "brl_hand_posterior_smc")
 OPS = (
     "brl_make_keys", "brl_init", "brl_reset_fields", "brl_step", "brl_duplicate_step", "brl_duplicate_init",
     "brl_observe", "brl_legal_mask", "brl_rollout_random", "brl_imp_reward", "brl_gae", "brl_categorical",
@@ -37,7 +37,7 @@ MISC = ("brl_last_error", "brl_abi_version", "brl_mlp_packed_bytes", "brl_mlp_sc
         "brl_duplicate_match_scratch_bytes", "brl_duplicate_match_graph_builds", "brl_evaluate_match_scratch_bytes",
         "brl_evaluate_match_partner_scratch_bytes",
         "brl_ppo_grad_grouped_scratch_bytes", "brl_mlp_param_stride", "brl_call_values_scratch_bytes",
-        "brl_hand_posterior_scratch_bytes")
+        "brl_hand_posterior_scratch_bytes", "brl_hand_posterior_smc_scratch_bytes")
 XLA_LEGACY = tuple(op + "_xla" for op in OPS)  # legacy XLA GPU custom-call targets (csrc/xla_ffi_shim.cc)
 ALL_SYMBOLS = OPS + HOST_API + MISC + XLA_LEGACY
 
@@ -69,7 +69,9 @@ F_PLAYER_MODELS = 1 << 24  # brl_model_rows / brl_duplicate_match: env_models[n,
 SYS_CONTEXTS, SYS_COLS = 75, 96  # the bidding-system histogram hist[M, 75, 38, 96] (BRL_SYS_*)
 # brl_hand_posterior's per-query status codes (BRL_POST_*) and its Philox stream tag
 POST_OK, POST_ILLEGAL, POST_SHORT, POST_BAD_NET, POST_BAD_QUERY, POST_CAPACITY = 0, 1, 2, 3, 4, 5
+POST_STAGES = 6  # brl_hand_posterior_smc: the prefix is longer than the stage bound
 POST_TAG = 0x484E4430
+SMC_TAG, SMC_MAX_MOVES, SMC_MAX_STAGES = 0x534D0000, 64, 320  # brl_hand_posterior_smc (BRL_SMC_*)
 POST_FEATURES = 95
 
 
@@ -94,6 +96,11 @@ class BrlParams(C.Structure):
         ("n_deals", C.c_int32), ("flags", C.c_int32), ("step", C.c_uint32), ("k_steps", C.c_int32),
         ("illegal_penalty", C.c_float), ("illegal_bonus", C.c_float), ("gamma", C.c_float), ("gae_lambda", C.c_float),
     ]
+
+
+class BrlSmcParams(C.Structure):
+    _fields_ = [("post", BrlParams), ("ess_threshold", C.c_float), ("moves", C.c_int32), ("stages", C.c_int32),
+                ("reserved", C.c_int32)]
 
 
 class BrlPpoParams(C.Structure):

@@ -827,9 +827,11 @@ int32_t brl_duplicate_match(brl_stream_t stream, void** b, const void* opaque, s
                                     "status", BRL_TABLE_INFO_NAMES, "system histogram [21]"};
     static const uint8_t align[22] = {16, 16, 16, 8, 8, 16, 4, 8, 4, 0, 16, 0, 0, 0, 0, 0, 16, 0, 0, 0, 0, 4};
     const unsigned nullable = 1u << 3 | 1u << 4 | 0xFFFu << 9 | 1u << 21;
-    if ((rc = check_buffers("brl_duplicate_match", b, names, 22, nullable, 0u, align))) return rc;
+    // problems are reported in buffer order: the Table_info group [9..20] before the optional histogram [21]
+    if ((rc = check_buffers("brl_duplicate_match", b, names, 21, nullable, 0u, align))) return rc;
     const int tables = given(b, 9, 21);
     if (tables != 0 && tables != 12) return fail(BRL_E_BUFFER, "brl_duplicate_match: give all twelve Table_info buffers [9..20] or none");
+    if ((rc = check_buffers("brl_duplicate_match", b, names, 22, nullable, 0u, align))) return rc;
 
     MatchPlan q = base_plan("brl_duplicate_match", 0, p, M, b[5]);
     q.P = P;
@@ -946,9 +948,11 @@ int32_t brl_call_values(brl_stream_t stream, void** b, const void* opaque, size_
                                     "regret_sums", "mismatch", "status", "count", "env", "table", "player", "net", "context", "played",
                                     "r", "obs", "gain"};
     static const uint8_t align[21] = {16, 0, 16, 16, 16, 16, 16, 8, 8, 8, 4, 8, 4, 4, 4, 4, 4, 4, 4, 16, 4};
-    if ((rc = check_buffers("brl_call_values", b, names, 21, 0x3FFu << 11, 0u, align))) return rc;
+    // problems are reported in buffer order: the record group [11..18] before the optional examples [19], [20]
+    if ((rc = check_buffers("brl_call_values", b, names, 19, 0x3FFu << 11, 0u, align))) return rc;
     const int records = given(b, 11, 19);
     if (records != 0 && records != 8) return fail(BRL_E_BUFFER, "brl_call_values: give all eight record buffers [11..18] or none");
+    if ((rc = check_buffers("brl_call_values", b, names, 21, 0x3FFu << 11, 0u, align))) return rc;
     const bool examples = b[19] != nullptr;
     if (examples != (b[20] != nullptr))
         return fail(BRL_E_BUFFER, "brl_call_values: give both training-example buffers [19] obs and [20] gain, or neither");

@@ -89,6 +89,7 @@
     X(brl_cv_grad, "iisioos") \
     X(brl_cv_eval, "iisios") \
     X(brl_hand_posterior, "iiiiiiiiisoooo") \
+    X(brl_hand_posterior_smc, "iiiiiiiiisooooooo") \
     /* end */
 
 namespace {

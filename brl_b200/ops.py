@@ -1046,23 +1046,12 @@ def hand_posterior_scratch_bytes(n_queries: int, n_samples: int, row_capacity: i
     return _size_query("brl_hand_posterior_scratch_bytes", n_queries, n_samples, row_capacity, n_models)
 
 
-def hand_posterior(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tensor, query: torch.Tensor, seat_nets: torch.Tensor,
-                   pool: torch.Tensor, scratch: torch.Tensor, cards: torch.Tensor, features: torch.Tensor, weights: torch.Tensor,
-                   status: torch.Tensor, *, samples: int, row_capacity: int, board: Optional[torch.Tensor] = None,
-                   dealer: Optional[torch.Tensor] = None, vul: Optional[torch.Tensor] = None, seed: int = 0, query_offset: int = 0,
-                   temperature: float = 1.0, single_bf16: bool = False, path_flags: int = 0, hands: Optional[torch.Tensor] = None,
-                   logw: Optional[torch.Tensor] = None) -> None:
-    """The posterior of the hidden hands for Q queries (brl_hand_posterior, DESIGN.md f18): query[j] = (t, s, L) reads the first L
-    calls of auction t (calls[offsets[t]:offsets[t + 1]], u8 0..37, on deal row board[t] (None: row t), dealer dealer[t] (int8;
-    None: North), vulnerability vul[t] (u8, bit 0 NS, bit 1 EW; None: none)) from absolute seat s, with net seat_nets[j, seat]
-    (int32 [Q, 4]) of `pool` at each seat.  Writes cards f64[Q, 3, 52], features f64[Q, 3, 95], weights f64[Q, 4] and status
-    int32[Q]; hands u64 (int64) [Q, N, 4] and logw f64[Q, N] are optional diagnostics, both or neither.  `row_capacity` (a
-    multiple of 256) sizes the forward; the scratch is hand_posterior_scratch_bytes(Q, N, row_capacity, M) bytes.  Every
-    argument is checked on the host (one device-to-host copy of offsets, calls and query) before any device work."""
-    who = "hand_posterior"
+def _check_posterior(who, table, calls, offsets, query, seat_nets, pool, scratch, outputs, *, N, row_capacity, board, dealer, vul,
+                     temperature, path_flags, diagnostics, scratch_bytes):
+    """the host checks of hand_posterior / hand_posterior_smc, in order; outputs and diagnostics: [(name, tensor, shape, dtype)]
+    (the diagnostics all or none) -> Q, or None for an empty batch"""
     n = int(offsets.shape[0]) - 1 if offsets.dim() == 1 else -1
     Q = int(query.shape[0]) if query.dim() == 2 else -1
-    N = int(samples)
     if offsets.dtype != torch.int64 or n < 0:
         raise _lib.BrlError(f"{who}: offsets must be int64 [n + 1]")
     if calls.dtype != torch.uint8 or calls.dim() != 1:
@@ -1085,20 +1074,21 @@ def hand_posterior(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tens
         raise _lib.BrlError(f"{who}: temperature must be finite and >= 0")
     if path_flags & ~(_lib.F_TUNE_MLP_LAYERS | _lib.F_TUNE_MLP_FUSED):
         raise _lib.BrlError(f"{who}: path_flags may hold F_TUNE_MLP_LAYERS / F_TUNE_MLP_FUSED only")
-    for name, t, shape, dt in (("cards", cards, (Q, 3, 52), torch.float64), ("features", features, (Q, 3, _lib.POST_FEATURES), torch.float64),
-                               ("weights", weights, (Q, 4), torch.float64), ("status", status, (Q,), torch.int32)):
+    for name, t, shape, dt in outputs(Q):
         if t.dtype != dt or tuple(t.shape) != shape:
             raise _lib.BrlError(f"{who}: {name} must be {str(dt).replace('torch.', '')} {list(shape)}")
-    if (hands is None) != (logw is None):
-        raise _lib.BrlError(f"{who}: hands and logw go together")
-    if hands is not None and (hands.dtype != torch.int64 or tuple(hands.shape) != (Q, N, 4) or logw.dtype != torch.float64
-                              or tuple(logw.shape) != (Q, N)):
-        raise _lib.BrlError(f"{who}: hands must be int64 [Q, N, 4] and logw float64 [Q, N]")
+    for group in diagnostics(Q):
+        names = " and ".join(name for name, *_ in group)
+        if len({t is None for _n, t, _s, _d in group}) > 1:
+            raise _lib.BrlError(f"{who}: {names} go together")
+        if group[0][1] is not None and any(t.dtype != dt or tuple(t.shape) != shape for _n, t, shape, dt in group):
+            raise _lib.BrlError(f"{who}: " + ", ".join(f"{name} must be {str(dt).replace('torch.', '')} {list(shape)}"
+                                                     for name, _t, shape, dt in group))
     if Q == 0:
-        return
-    need = hand_posterior_scratch_bytes(Q, N, row_capacity, M)
+        return None
+    need = scratch_bytes(Q, N, row_capacity, M)
     if scratch.dtype != torch.uint8 or scratch.dim() != 1 or scratch.numel() < need:
-        raise _lib.BrlError(f"{who}: scratch must be u8 [>= {need}] (hand_posterior_scratch_bytes)")
+        raise _lib.BrlError(f"{who}: scratch must be u8 [>= {need}] ({who}_scratch_bytes)")
     off, q, c = offsets.cpu(), query.cpu(), calls.cpu()
     if int(off[0]) != 0 or bool((off[1:] < off[:-1]).any()) or int(off[-1]) != calls.shape[0]:
         raise _lib.BrlError(f"{who}: offsets must rise from 0 to len(calls)")
@@ -1108,9 +1098,105 @@ def hand_posterior(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tens
         raise _lib.BrlError(f"{who}: a query's auction is outside [0, {n})")
     if board is None and n > table.shape[0]:
         raise _lib.BrlError(f"{who}: without board auction t needs deal row t: the table is too short")
+    return Q
+
+
+def _posterior_outputs(cards, features, weights, status):
+    return lambda Q: (("cards", cards, (Q, 3, 52), torch.float64), ("features", features, (Q, 3, _lib.POST_FEATURES), torch.float64),
+                      ("weights", weights, (Q, 4), torch.float64), ("status", status, (Q,), torch.int32))
+
+
+def hand_posterior(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tensor, query: torch.Tensor, seat_nets: torch.Tensor,
+                   pool: torch.Tensor, scratch: torch.Tensor, cards: torch.Tensor, features: torch.Tensor, weights: torch.Tensor,
+                   status: torch.Tensor, *, samples: int, row_capacity: int, board: Optional[torch.Tensor] = None,
+                   dealer: Optional[torch.Tensor] = None, vul: Optional[torch.Tensor] = None, seed: int = 0, query_offset: int = 0,
+                   temperature: float = 1.0, single_bf16: bool = False, path_flags: int = 0, hands: Optional[torch.Tensor] = None,
+                   logw: Optional[torch.Tensor] = None) -> None:
+    """The posterior of the hidden hands for Q queries (brl_hand_posterior, DESIGN.md f18): query[j] = (t, s, L) reads the first L
+    calls of auction t (calls[offsets[t]:offsets[t + 1]], u8 0..37, on deal row board[t] (None: row t), dealer dealer[t] (int8;
+    None: North), vulnerability vul[t] (u8, bit 0 NS, bit 1 EW; None: none)) from absolute seat s, with net seat_nets[j, seat]
+    (int32 [Q, 4]) of `pool` at each seat.  Writes cards f64[Q, 3, 52], features f64[Q, 3, 95], weights f64[Q, 4] and status
+    int32[Q]; hands u64 (int64) [Q, N, 4] and logw f64[Q, N] are optional diagnostics, both or neither.  `row_capacity` (a
+    multiple of 256) sizes the forward; the scratch is hand_posterior_scratch_bytes(Q, N, row_capacity, M) bytes.  Every
+    argument is checked on the host (one device-to-host copy of offsets, calls and query) before any device work."""
+    N = int(samples)
+    Q = _check_posterior("hand_posterior", table, calls, offsets, query, seat_nets, pool, scratch,
+                         _posterior_outputs(cards, features, weights, status), N=N, row_capacity=row_capacity, board=board,
+                         dealer=dealer, vul=vul, temperature=temperature, path_flags=path_flags,
+                         diagnostics=lambda Q: [[("hands", hands, (Q, N, 4), torch.int64), ("logw", logw, (Q, N), torch.float64)]],
+                         scratch_bytes=hand_posterior_scratch_bytes)
+    if Q is None:
+        return
     flags = (F_MLP_BF16 if single_bf16 else 0) | int(path_flags)
     _call("brl_hand_posterior",
           [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(board), _ptr(dealer), _ptr(vul), _ptr(query), _ptr(seat_nets), _ptr(pool),
            _ptr(scratch), _ptr(cards), _ptr(features), _ptr(weights), _ptr(status), _ptr(hands), _ptr(logw)],
-          BrlParams(Q, int(query_offset), int(row_capacity), int(seed) & 0xFFFFFFFFFFFFFFFF, int(table.shape[0]), flags, N, M,
-                    -1.0, 1.0, float(temperature), 0.0))  # BrlParams directly: _params would turn a capacity of 0 into Q
+          BrlParams(Q, int(query_offset), int(row_capacity), int(seed) & 0xFFFFFFFFFFFFFFFF, int(table.shape[0]), flags, N,
+                    int(pool.shape[0]), -1.0, 1.0, float(temperature), 0.0))  # BrlParams directly: _params would turn a capacity of 0 into Q
+
+
+# ---- hand reading by resample-move SMC (DESIGN.md f19) ----------------------------------------------------------------------
+def hand_posterior_smc_scratch_bytes(n_queries: int, n_samples: int, row_capacity: int, n_models: int) -> int:
+    return _size_query("brl_hand_posterior_smc_scratch_bytes", n_queries, n_samples, row_capacity, n_models)
+
+
+SMC_TRACE = ("loglik", "ancestors", "pairs", "accepted", "proposed")
+
+
+def smc_trace(Q: int, N: int, stages: int, moves: int, device) -> dict:
+    """empty trace buffers of brl_hand_posterior_smc: loglik f64[Q, K, N], ancestors i32[Q, K, N], pairs i32[Q, K, R],
+    accepted u8[Q, K, R, N], proposed f64[Q, K, R, N, 2]"""
+    K, R = int(stages), int(moves)
+    return dict(loglik=torch.empty((Q, K, N), dtype=torch.float64, device=device),
+                ancestors=torch.empty((Q, K, N), dtype=torch.int32, device=device),
+                pairs=torch.empty((Q, K, R), dtype=torch.int32, device=device),
+                accepted=torch.empty((Q, K, R, N), dtype=torch.uint8, device=device),
+                proposed=torch.empty((Q, K, R, N, 2), dtype=torch.float64, device=device))
+
+
+def hand_posterior_smc(table: torch.Tensor, calls: torch.Tensor, offsets: torch.Tensor, query: torch.Tensor, seat_nets: torch.Tensor,
+                       pool: torch.Tensor, scratch: torch.Tensor, cards: torch.Tensor, features: torch.Tensor, weights: torch.Tensor,
+                       status: torch.Tensor, log_evidence: torch.Tensor, resamples: torch.Tensor, acceptance: torch.Tensor, *,
+                       samples: int, row_capacity: int, stages: int, moves: int = 1, ess_threshold: float = 0.5,
+                       board: Optional[torch.Tensor] = None, dealer: Optional[torch.Tensor] = None,
+                       vul: Optional[torch.Tensor] = None, seed: int = 0, query_offset: int = 0, temperature: float = 1.0,
+                       single_bf16: bool = False, path_flags: int = 0, hands: Optional[torch.Tensor] = None,
+                       logw: Optional[torch.Tensor] = None, ell: Optional[torch.Tensor] = None,
+                       trace: Optional[dict] = None) -> None:
+    """The posterior of hand_posterior by resample-move SMC over the calls of each prefix (brl_hand_posterior_smc, DESIGN.md
+    f19).  Arguments and outputs as hand_posterior, plus log_evidence f64[Q], resamples int32[Q] and acceptance f64[Q];
+    `stages` >= every query's L (a longer prefix gets POST_STAGES), `moves` in [0, 64] Metropolis-Hastings moves after each
+    resample, `ess_threshold` kappa in [0, 1] (resample when ESS < kappa N; 1 resamples at every stage).  `row_capacity`
+    bounds each stage's and each move's forward.  Optional: hands / logw / ell f64[Q, N, 3] (the final particles, all or
+    none) and `trace` (smc_trace's five buffers, all or none).  Every argument is checked before any device work."""
+    who, N, K, R = "hand_posterior_smc", int(samples), int(stages), int(moves)
+    if not 0 <= R <= _lib.SMC_MAX_MOVES:
+        raise _lib.BrlError(f"{who}: moves must be in [0, {_lib.SMC_MAX_MOVES}]")
+    if not 0 <= K <= _lib.SMC_MAX_STAGES:
+        raise _lib.BrlError(f"{who}: stages must be in [0, {_lib.SMC_MAX_STAGES}]")
+    if not 0.0 <= ess_threshold <= 1.0:
+        raise _lib.BrlError(f"{who}: ess_threshold must be in [0, 1]")
+    tr = trace or {}
+    if trace is not None and set(trace) != set(SMC_TRACE):
+        raise _lib.BrlError(f"{who}: trace must hold {', '.join(SMC_TRACE)}")
+    base = _posterior_outputs(cards, features, weights, status)
+    outputs = lambda Q: base(Q) + (("log_evidence", log_evidence, (Q,), torch.float64), ("resamples", resamples, (Q,), torch.int32),  # noqa: E731
+                                   ("acceptance", acceptance, (Q,), torch.float64))
+    diagnostics = lambda Q: [  # noqa: E731
+        [("hands", hands, (Q, N, 4), torch.int64), ("logw", logw, (Q, N), torch.float64), ("ell", ell, (Q, N, 3), torch.float64)],
+        [("trace loglik", tr.get("loglik"), (Q, K, N), torch.float64), ("trace ancestors", tr.get("ancestors"), (Q, K, N), torch.int32),
+         ("trace pairs", tr.get("pairs"), (Q, K, R), torch.int32), ("trace accepted", tr.get("accepted"), (Q, K, R, N), torch.uint8),
+         ("trace proposed", tr.get("proposed"), (Q, K, R, N, 2), torch.float64)]]
+    Q = _check_posterior(who, table, calls, offsets, query, seat_nets, pool, scratch, outputs, N=N, row_capacity=row_capacity,
+                         board=board, dealer=dealer, vul=vul, temperature=temperature, path_flags=path_flags,
+                         diagnostics=diagnostics, scratch_bytes=hand_posterior_smc_scratch_bytes)
+    if Q is None:
+        return
+    flags = (F_MLP_BF16 if single_bf16 else 0) | int(path_flags)
+    post = BrlParams(Q, int(query_offset), int(row_capacity), int(seed) & 0xFFFFFFFFFFFFFFFF, int(table.shape[0]), flags, N,
+                     int(pool.shape[0]), -1.0, 1.0, float(temperature), 0.0)
+    _call("brl_hand_posterior_smc",
+          [_ptr(table), _ptr(calls), _ptr(offsets), _ptr(board), _ptr(dealer), _ptr(vul), _ptr(query), _ptr(seat_nets), _ptr(pool),
+           _ptr(scratch), _ptr(cards), _ptr(features), _ptr(weights), _ptr(status), _ptr(log_evidence), _ptr(resamples),
+           _ptr(acceptance), _ptr(hands), _ptr(logw), _ptr(ell)] + [_ptr(tr.get(k)) for k in SMC_TRACE],
+          _lib.BrlSmcParams(post, float(ess_threshold), R, K, 0))

@@ -3,7 +3,9 @@ policies, and how much hand information a net's auctions carry.
 
 `hand_posterior` runs brl_hand_posterior: for each query (auction, observer seat, prefix length) it deals the 39 unseen cards
 at random N times, weights every deal by the probability that the nets would have made the other seats' calls with those
-hands, and returns the weighted card holdings and hand features.  `describe` prints one query's posterior, and `hand_reading`
+hands, and returns the weighted card holdings and hand features.  With method="smc" it runs brl_hand_posterior_smc instead
+(DESIGN.md f19): the same deals are reweighted call by call, resampled when their effective sample size falls below
+ess_threshold x N, and moved by Metropolis-Hastings card swaps, so long auctions keep usable samples.  `describe` prints one query's posterior, and `hand_reading`
 scores the posteriors of auctions whose deals are known."""
 from __future__ import annotations
 
@@ -41,43 +43,93 @@ def query_segments(queries: np.ndarray, seat_nets: np.ndarray, dealers: np.ndarr
     return out
 
 
+def smc_segments(queries: np.ndarray, seat_nets: np.ndarray, dealers: np.ndarray, moves: bool) -> List[Dict]:
+    """per query of brl_hand_posterior_smc: {forward: {net: calls}} over the forwards it takes part in, ("w", k) for stage k's
+    reweight and, with moves, ("m", k) for the moves after a resample at stage k, at the most rows any pair of hidden seats
+    can need; a chunk's forward capacity is the largest of these forwards summed over its queries"""
+    out = []
+    for (t, s, L), nets, d in zip(queries, seat_nets, dealers):
+        seg: Dict = {}
+        by_seat = [0, 0, 0, 0]
+        if 0 <= s < 4:
+            for k in range(int(L)):
+                caller = (int(d) + k) % 4
+                if caller == s:
+                    continue
+                by_seat[caller] += 1
+                seg[("w", k)] = {int(nets[caller]): 1}
+                if moves:
+                    bound: Dict[int, int] = {}
+                    hidden = [(int(s) + 1 + r) % 4 for r in range(3)]
+                    for a, b in ((0, 1), (0, 2), (1, 2)):
+                        pair: Dict[int, int] = {}
+                        for seat in (hidden[a], hidden[b]):
+                            if by_seat[seat]:
+                                pair[int(nets[seat])] = pair.get(int(nets[seat]), 0) + by_seat[seat]
+                        for m, n in pair.items():
+                            bound[m] = max(bound.get(m, 0), n)
+                    seg[("m", k)] = bound
+        out.append(seg)
+    return out
+
+
 def _padded(per_net: Dict[int, int], N: int) -> int:
     return sum((N * n + 255) // 256 * 256 for n in per_net.values())
 
 
-def pack_chunks(segments: Sequence[Dict[int, int]], N: int, row_budget: int):
+def pack_chunks(segments: Sequence[Dict], N: int, row_budget: int):
     """Consecutive query ranges [(begin, end, padded rows)] whose forward fits `row_budget` rows; a query that does not fit
-    alone raises ValueError with the budget it needs."""
+    alone raises ValueError with the budget it needs.  segments[j] is query_segments' {net: calls} (one forward), or
+    smc_segments' {forward: {net: calls}}: then the rows of a chunk are those of its largest forward, not their sum."""
+    def rows(acc):
+        return max((_padded(v, N) for v in acc.values()), default=0)
+
+    def add(acc, seg):
+        out = {key: dict(v) for key, v in acc.items()}
+        for key, per_net in seg.items():
+            tot = out.setdefault(key, {})
+            for m, n in per_net.items():
+                tot[m] = tot.get(m, 0) + n
+        return out
+
+    staged = [seg if seg and isinstance(next(iter(seg.values())), dict) else {0: seg} for seg in segments]
     chunks, begin, acc = [], 0, {}
-    for j, seg in enumerate(segments):
-        alone = _padded(seg, N)
+    for j, seg in enumerate(staged):
+        alone = rows(seg)
         if alone > row_budget:
+            calls = max((sum(v.values()) for v in seg.values()), default=0)
             raise ValueError(f"hand_posterior: query {j} needs a row_budget of at least {alone} rows ({N} samples x "
-                             f"{sum(seg.values())} calls by other seats), the budget is {row_budget}")
-        trial = dict(acc)
-        for m, n in seg.items():
-            trial[m] = trial.get(m, 0) + n
-        if j > begin and _padded(trial, N) > row_budget:
-            chunks.append((begin, j, _padded(acc, N)))
-            begin, trial = j, dict(seg)
+                             f"{calls} calls by other seats), the budget is {row_budget}")
+        trial = add(acc, seg)
+        if j > begin and rows(trial) > row_budget:
+            chunks.append((begin, j, rows(acc)))
+            begin, trial = j, add({}, seg)
         acc = trial
-    if begin < len(segments):
-        chunks.append((begin, len(segments), _padded(acc, N)))
+    if begin < len(staged):
+        chunks.append((begin, len(staged), rows(acc)))
     return chunks
 
 
 def hand_posterior(params_list, table, calls, offsets, queries, seat_nets, *, board=None, dealer=None, vul=None, samples: int = 1024,
                    seed: int = 0, temperature: float = 1.0, precision: Optional[str] = None, row_budget: int = DEFAULT_ROW_BUDGET,
-                   diagnostics: bool = False, path_flags: int = 0, device="cuda") -> Dict[str, np.ndarray]:
+                   diagnostics: bool = False, path_flags: int = 0, method: str = "is", moves: int = 1, ess_threshold: float = 0.5,
+                   device="cuda") -> Dict[str, np.ndarray]:
     """Posterior of the hidden hands for every query (t, s, L) of `queries` (int [Q, 3]): auction t of calls / offsets (u8 /
     int64, brl_sl_examples' encoding) read by absolute seat s after its first L calls, seat k playing net seat_nets[j, k] of
     params_list.  board / dealer / vul as ops.hand_posterior (None: row t, North, nobody vulnerable).  Queries are packed into
     device calls of at most `row_budget` forward rows; sample i of query j depends on (seed, j, i) only.
     -> numpy: cards [Q, 3, 52] and features [Q, 3, 95] (relative seats LHO, partner, RHO), ess [Q], accepted [Q] (samples with
     weight > 0), log_max [Q], weights [Q, 4], status [Q] (BRL_POST_*), and with diagnostics hands [Q, N, 4] (u64 masks by absolute
-    seat) and logw [Q, N]."""
+    seat) and logw [Q, N].
+    method="smc" runs the resample-move sequential Monte Carlo sampler (ops.hand_posterior_smc) with `moves` Metropolis-Hastings
+    moves after each resample and resampling when the ESS falls below ess_threshold x N; the result gains log_evidence [Q],
+    resamples [Q] and acceptance [Q] (and ell [Q, N, 3] with diagnostics).  Chunks are then sized by the largest forward of
+    any stage or move."""
     if precision not in (None, "tc", "tc-bf16"):
         raise ValueError(f"unknown precision {precision!r}")
+    if method not in ("is", "smc"):
+        raise ValueError(f"unknown method {method!r}: 'is' or 'smc'")
+    smc = method == "smc"
     if not params_list:
         raise ValueError("hand_posterior: no nets")
     queries = np.ascontiguousarray(queries, dtype=np.int32).reshape(-1, 3)
@@ -90,7 +142,10 @@ def hand_posterior(params_list, table, calls, offsets, queries, seat_nets, *, bo
         raise ValueError(f"hand_posterior: a query's auction is outside [0, {n_auctions})")
     N, Q = int(samples), queries.shape[0]
     dealers = np.zeros(n_auctions, np.int64) if dealer is None else np.asarray(dealer, np.int64)
-    chunks = pack_chunks(query_segments(queries, seat_nets, dealers[queries[:, 0]] if Q else np.zeros(0, np.int64)), N, row_budget)
+    qd = dealers[queries[:, 0]] if Q else np.zeros(0, np.int64)
+    segments = (smc_segments(queries, seat_nets, qd, moves > 0 and ess_threshold > 0) if smc
+                else query_segments(queries, seat_nets, qd))
+    chunks = pack_chunks(segments, N, row_budget)
     dev = torch.device(device)
 
     def t(a, dt):
@@ -103,19 +158,33 @@ def hand_posterior(params_list, table, calls, offsets, queries, seat_nets, *, bo
                status=np.zeros(Q, np.int32))
     if diagnostics:
         out["hands"], out["logw"] = np.zeros((Q, N, 4), np.uint64), np.zeros((Q, N))
+    if smc:
+        out.update(log_evidence=np.full(Q, np.nan), resamples=np.zeros(Q, np.int32), acceptance=np.full(Q, np.nan))
+        if diagnostics:
+            out["ell"] = np.zeros((Q, N, 3))
     for b, e, rows in chunks:
         q = e - b
-        scratch = torch.empty(ops.hand_posterior_scratch_bytes(q, N, rows, pool.shape[0]), dtype=torch.uint8, device=dev)
+        size = (ops.hand_posterior_smc_scratch_bytes if smc else ops.hand_posterior_scratch_bytes)(q, N, rows, pool.shape[0])
+        scratch = torch.empty(size, dtype=torch.uint8, device=dev)
         res = dict(cards=torch.empty((q, 3, 52), dtype=torch.float64, device=dev),
                    features=torch.empty((q, 3, _lib.POST_FEATURES), dtype=torch.float64, device=dev),
                    weights=torch.empty((q, 4), dtype=torch.float64, device=dev), status=torch.empty(q, dtype=torch.int32, device=dev))
         diag = {}
         if diagnostics:
             diag = dict(hands=torch.empty((q, N, 4), dtype=torch.int64, device=dev), logw=torch.empty((q, N), dtype=torch.float64, device=dev))
-        ops.hand_posterior(table_t, calls_t, offsets_t, t(queries[b:e], np.int32), t(seat_nets[b:e], np.int32), pool, scratch,
-                           res["cards"], res["features"], res["weights"], res["status"], samples=N, row_capacity=rows, board=board_t,
-                           dealer=dealer_t, vul=vul_t, seed=seed, query_offset=b, temperature=temperature,
-                           single_bf16=precision == "tc-bf16", path_flags=path_flags, **diag)
+        args = (table_t, calls_t, offsets_t, t(queries[b:e], np.int32), t(seat_nets[b:e], np.int32), pool, scratch, res["cards"],
+                res["features"], res["weights"], res["status"])
+        kw = dict(samples=N, row_capacity=rows, board=board_t, dealer=dealer_t, vul=vul_t, seed=seed, query_offset=b,
+                  temperature=temperature, single_bf16=precision == "tc-bf16", path_flags=path_flags, **diag)
+        if smc:
+            res.update(log_evidence=torch.empty(q, dtype=torch.float64, device=dev), resamples=torch.empty(q, dtype=torch.int32, device=dev),
+                       acceptance=torch.empty(q, dtype=torch.float64, device=dev))
+            if diagnostics:
+                diag["ell"] = kw["ell"] = torch.empty((q, N, 3), dtype=torch.float64, device=dev)
+            ops.hand_posterior_smc(*args, res["log_evidence"], res["resamples"], res["acceptance"],
+                                   stages=int(queries[b:e, 2].max(initial=0)), moves=moves, ess_threshold=ess_threshold, **kw)
+        else:
+            ops.hand_posterior(*args, **kw)
         for k, v in res.items():
             out[k][b:e] = v.cpu().numpy()
         for k, v in diag.items():
@@ -207,13 +276,18 @@ def reading_stats(post: Dict[str, np.ndarray], queries: np.ndarray, seat_nets: n
             partner_cards_read=float(np.mean(a["partner"])) if ok else None, partner_cards_read_prior=13.0 / 3.0,
             hcp_abs_error={name: (float(err[:, r].mean()) if ok else None) for r, name in enumerate(REL_NAMES)},
             ess_quantiles={f"p{q}": (float(np.percentile(a["ess"], q)) if ok else None) for q in (10, 50, 90)})
+        if "acceptance" in post:  # SMC: the mean Metropolis-Hastings acceptance over the queries that moved
+            acc = [float(post["acceptance"][j]) for j in range(len(queries)) if int(seat_nets[j, int(queries[j, 1])]) == net
+                   and np.isfinite(post["acceptance"][j])]
+            report[str(net)]["acceptance_mean"] = float(np.mean(acc)) if acc else None
     return report
 
 
 def hand_reading(params_list, table, calls, offsets, seat_nets_by_auction, *, board=None, dealer=None, vul=None, at: str = "end",
                  **kwargs) -> Dict[str, Dict]:
     """The hand-reading report of auctions with known deals: every auction read by each seat (reading_queries), the posterior
-    of hand_posterior (kwargs: samples, seed, temperature, precision, row_budget), scored by reading_stats per observer net."""
+    of hand_posterior (kwargs: samples, seed, temperature, precision, row_budget, method, moves, ess_threshold), scored by
+    reading_stats per observer net."""
     queries, seat_nets = reading_queries(offsets, seat_nets_by_auction, dealer, at)
     post = hand_posterior(params_list, table, calls, offsets, queries, seat_nets, board=board, dealer=dealer, vul=vul, **kwargs)
     owners, _ = unpack_deal_table(table)

@@ -66,6 +66,8 @@
  *                         tensor-core forward / backward of brl_sl_grad (DESIGN.md f17)
  *   brl_hand_posterior    not in the reference: the hidden hands an auction implies under the nets' policies, by importance
  *                         sampling of the unseen cards with the grouped forward as the likelihood (DESIGN.md f18)
+ *   brl_hand_posterior_smc  not in the reference: the same posterior by resample-move sequential Monte Carlo over the calls
+ *                         of the auction (DESIGN.md f19)
  *   brl_eval_act_log      make_action + make_step_log of evaluate / duplicate_evaluate   src/evaluation.py:236-385, 650-745
  *   brl_eval_summary      make_terminated_log + the log_info means                        src/evaluation.py:448-596, 839-1027
  *   brl_mlp_pack          the params pytree (bridge_models/<name>.pkl, ppo.py:351-362) -> device layout
@@ -549,6 +551,54 @@ int32_t brl_call_values(brl_stream_t, void **buffers, const void *opaque, size_t
 int64_t brl_hand_posterior_scratch_bytes(int64_t n_queries, int64_t n_samples, int64_t row_capacity, int64_t n_models);
 int32_t brl_hand_posterior(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
 
+/* ---- hand reading by resample-move SMC (not in the reference; DESIGN.md f19, restated by tests/smc_ref.py) ---------------
+ * The query of brl_hand_posterior, answered by sequential Monte Carlo over the calls of the prefix (Gilks & Berzuini 2001;
+ * Del Moral, Doucet & Jasra 2006), so that long and informative auctions keep an effective sample size.
+ *   Particles i = 0..N-1 of query g start as brl_hand_posterior's samples; each carries its hidden hands, log w (f64, 0) and
+ *   ell[r] (f64, 0), the sum of its l_k over the calls of hidden seat r (0 LHO, 1 partner, 2 RHO).  Stage k = 0 .. K-1
+ *   (K = `stages` >= every query's L): a stage with k >= L, a call by the observer, or an extinct query does nothing.  Else,
+ *   sigma_k the caller:
+ *   1. reweight: l_k is brl_hand_posterior's term of call k on the particle's hands; log w += l_k, ell[sigma_k] += l_k.
+ *   2. resample: M = max log w; if M = -inf the query is extinct for good.  w' = exp(log w - M), W = sum w', S = sum w'^2 (i
+ *      increasing).  When kappa = 1 or W * W / S < kappa * N: systematic resampling with u = (x + 0.5) 2^-32, x = word x of
+ *      philox4x32(counter (g_lo, g_hi, BRL_SMC_TAG + 128 k, 0xFFFFFFFF), key (seed_lo, seed_hi)): C_m = C_{m-1} + w'_m (i
+ *      increasing, C_0 = w'_0); the ancestor of particle i is the first m with C_m >= (i + u) * W / N (at most N - 1).  Hands
+ *      and ell are copied from the ancestors, log_evidence += log(W / N) + M, log w = 0, resamples += 1.
+ *   3. move, after a resample only, for mv = 0 .. R-1: with P = philox4x32(counter (g_lo, g_hi, BRL_SMC_TAG + 128 k + 1 + mv,
+ *      c3), key): the pair is mulhi(P(c3 = 0xFFFFFFFF).x, 3) (0: LHO + partner, 1: LHO + RHO, 2: partner + RHO), shared by the
+ *      query; particle i (c3 = i) swaps card mulhi(P.x, 13) of r1 with card mulhi(P.y, 13) of r2 (the n-th card in increasing
+ *      card index).  ell'[r] = the sum of the proposed hands' l over seat r's calls at stages <= k (k increasing); accepted iff
+ *      log((P.z + 0.5) 2^-32) < (ell'[r1] + ell'[r2]) - (ell[r1] + ell[r2]), then hands and ell[r1], ell[r2] take the proposal.
+ *   4. end: brl_hand_posterior's reduction of log w; log_evidence += log(W / N) + M (-inf when nothing is accepted).
+ *   Every draw depends on (seed, g, k, mv, i) only, so results do not depend on batching.  With kappa = 0 no query resamples
+ *   and cards, features, weights, status, hands and log w are those of brl_hand_posterior bit for bit, on a pinned forward path.
+ * The call enqueues per stage: the row layout of call k of every live query, f18's public pass, expansion and grouped forward,
+ * the reweight, the ESS test / resampling (one thread per query), the gather; per move the proposal, the layout of the pair's
+ * calls at stages <= k for the queries that resampled, the forward and the MH test.  Row counts stay in device memory; no host
+ * synchronisation; capturable.  The row capacity bounds each forward, not their sum.
+ * buffers: [0]-[13] as brl_hand_posterior; [9] scratch (brl_hand_posterior_smc_scratch_bytes(Q, N, capacity, M))
+ *          [14] out f64 log_evidence[Q] (NaN on a status other than OK)  [15] out i32 resamples[Q]
+ *          [16] out f64 acceptance[Q] (accepted / proposed moves; NaN with none proposed)
+ *          [17] out u64 hands[Q, N, 4]  [18] out f64 logw[Q, N]  [19] out f64 ell[Q, N, 3] -- final particles, all or none
+ *          [20] out f64 trace_loglik[Q, K, N] (l_k, NaN when stage k does nothing)  [21] out i32 trace_ancestors[Q, K, N]
+ *          (-1 without a resample)  [22] out i32 trace_pairs[Q, K, R] (-1 without a move)  [23] out u8 trace_accepted[Q, K, R, N]
+ *          [24] out f64 trace_proposed[Q, K, R, N, 2] (ell'[r1], ell'[r2]) -- the trace, all five or none
+ * params: BrlSmcParams: post as brl_hand_posterior's BrlParams; ess_threshold = kappa in [0, 1]; moves = R in [0, 64];
+ *         stages = K in [0, 320]; reserved = 0.  A query with L > K gets BRL_POST_STAGES. */
+#define BRL_SMC_TAG 0x534D0000u  /* "SM": Philox stream of the SMC draws, + 128 k + (0 | 1 + mv) */
+#define BRL_POST_STAGES 6         /* brl_hand_posterior_smc: the prefix is longer than the stage bound */
+#define BRL_SMC_MAX_MOVES 64
+#define BRL_SMC_MAX_STAGES 320
+typedef struct BrlSmcParams {
+    BrlParams post;       /* brl_hand_posterior's parameters */
+    float ess_threshold;  /* kappa: resample when ESS < kappa N; 1 resamples at every stage */
+    int32_t moves;        /* R: Metropolis-Hastings moves after each resample */
+    int32_t stages;       /* K: the stage bound */
+    int32_t reserved;     /* 0 */
+} BrlSmcParams;
+int64_t brl_hand_posterior_smc_scratch_bytes(int64_t n_queries, int64_t n_samples, int64_t row_capacity, int64_t n_models);
+int32_t brl_hand_posterior_smc(brl_stream_t, void **buffers, const void *opaque, size_t opaque_len);
+
 /* ---- PPO update, non-GEMM part (src/update.py:74-242, ppo.py:195-211) ----------------------- */
 #define BRL_PPO_VALUE_CLIPPING  0x1 /* config["value_clipping"]  (src/update.py:47-62) */
 #define BRL_PPO_REWARD_SCALING  0x2 /* config["reward_scaling"]: (gae - mean) / (std + 1e-8) per minibatch (src/update.py:31-45) */
@@ -839,6 +889,7 @@ void brl_cv_grad_xla(brl_stream_t, void **buffers, const char *opaque, size_t op
 void brl_cv_eval_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_par_stats_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 void brl_hand_posterior_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
+void brl_hand_posterior_smc_xla(brl_stream_t, void **buffers, const char *opaque, size_t opaque_len, struct XlaCustomCallStatus_ *status);
 
 /* -------------------------------------------------------------------------
  * Host-buffer convenience layer (the call a non-JAX host makes): the library

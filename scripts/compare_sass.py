@@ -8,8 +8,9 @@ constant bank that holds the parameter block).  A refactor that changes template
 so kernels are paired by their demangled names after the renames in RENAMES; a rename to None marks a kernel the change
 removes on purpose.  Exit status 0 when every remaining kernel is identical and nothing else appeared or disappeared.
 
-RENAMES and ADDED record the hand-reading change (DESIGN.md f18): no kernel is renamed or removed, and the kernels of
-csrc/brl_posterior.cu (brl::k_post_*) are added.  Replace both tables for another change."""
+RENAMES and ADDED record the SMC hand-reading change (DESIGN.md f19): f18's segment-count and public-pass kernels became
+templates over the row set a forward reads, and f18's own row set (every call of the prefix) is the empty instantiation;
+the SMC kernels (brl::k_smc_*) and the SmcWindow instantiations are added.  Replace both tables for another change."""
 import argparse
 import os
 import re
@@ -18,8 +19,9 @@ import sys
 from collections import OrderedDict
 
 # (pattern, replacement) on names demangled as cu++filt prints them: template arguments read (int)128, (bool)1
-RENAMES = []
-ADDED = [r"^brl::k_post_"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
+RENAMES = [(r"^brl::k_post_count$", "brl::k_post_count<>"),
+           (r"^brl::k_post_public$", "brl::k_post_public<>")]
+ADDED = [r"^brl::k_smc_", r"^brl::k_post_(count|public)<brl::SmcWindow>$"]  # patterns of kernels the change adds on purpose: reported, not counted as unexpected
 
 
 def _cuobjdump(flag, lib):

@@ -1,7 +1,8 @@
 """Hand reading (DESIGN.md f18): how much each net's auctions tell its partner (and the opponents) about the hidden hands.
 
     python scripts/hand_reading.py [nets=a.pkl,b.pkl | seeds=1,2] [deals=dds_results/test_000.npy] boards=1000 \
-        [samples=1024] [temperature=1] [at=end|decisions] [precision=tc|tc-bf16] [out=hand_reading.json]
+        [samples=1024] [temperature=1] [at=end|decisions] [precision=tc|tc-bf16] [method=is|smc] [moves=1] \
+        [ess_threshold=0.5] [out=hand_reading.json]
     python scripts/hand_reading.py data=test.txt nets=a.pkl [max_auctions=1000] ...
     python scripts/hand_reading.py hand=AKQ2.AK32.K32.32 auction=1C,P,1H dealer=N vul=NS observer=S nets=a.pkl
 
@@ -9,7 +10,9 @@ Sources: a duplicate match of net 0 against net 1 (nets= .pkl files, or seeded n
 on `boards` boards of the deal table `deals=` (synthetic when omitted), both tables played by the host match loop with
 `record=`; or the auctions of an OpenSpiel data file (data=; dealer North, nobody vulnerable), every seat played by net 0.
 Every auction is read by each of its four seats (at=end: after the last call; at=decisions: before each of the seat's own
-calls) and scored per observer net (posterior.reading_stats).  Writes the JSON report.
+calls) and scored per observer net (posterior.reading_stats).  method=smc reads them with the resample-move SMC sampler
+(DESIGN.md f19: `moves` Metropolis-Hastings moves after each resample, resampling below ess_threshold x samples).  Writes the
+JSON report.
 
 With hand= (PBN order spades.hearts.diamonds.clubs, e.g. AKQ2.AK32.K32.32), auction= (comma-separated: P, X, XX, 1C .. 7NT),
 dealer=, vul= (None, NS, EW, Both) and observer= it prints posterior.describe for that one hand instead, every seat played by
@@ -25,7 +28,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."
 
 DEFAULTS = dict(nets="", seeds="1,2", deals="", boards=1000, data="", max_auctions=1000, samples=1024, seed=0, temperature=1.0,
                 at="end", precision="tc", row_budget=1 << 20, out="hand_reading.json", hand="", auction="", dealer="N",
-                vul="None", observer="S")
+                vul="None", observer="S", method="is", moves=1, ess_threshold=0.5)
 CALLS = ["P", "X", "XX"] + [f"{lvl}{s}" for lvl in range(1, 8) for s in ("C", "D", "H", "S", "NT")]
 RANKS = "23456789TJQKA"
 
@@ -41,6 +44,8 @@ def parse_args(argv):
         raise SystemExit("hand= and auction= go together")
     if cfg["at"] not in ("end", "decisions") or cfg["precision"] not in ("tc", "tc-bf16"):
         raise SystemExit("at= must be end or decisions, precision= tc or tc-bf16")
+    if cfg["method"] not in ("is", "smc") or not 0 <= cfg["moves"] <= 64 or not 0.0 <= cfg["ess_threshold"] <= 1.0:
+        raise SystemExit("method= must be is or smc, moves= in [0, 64], ess_threshold= in [0, 1]")
     return cfg
 
 
@@ -79,7 +84,8 @@ def main(argv):
     dev = "cuda"
     nets = load_nets(cfg, dev)
     kw = dict(samples=cfg["samples"], seed=cfg["seed"], temperature=cfg["temperature"], row_budget=cfg["row_budget"],
-              precision=None if cfg["precision"] == "tc" else cfg["precision"])
+              precision=None if cfg["precision"] == "tc" else cfg["precision"], method=cfg["method"], moves=cfg["moves"],
+              ess_threshold=cfg["ess_threshold"])
     if cfg["hand"]:
         table, calls, dealer, vul, s = one_hand_query(cfg)
         post = posterior.hand_posterior(nets[:1], table, np.array(calls, np.uint8), [0, len(calls)], [[0, s, len(calls)]],
